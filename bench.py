@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the 3DAHV hypothesis-and-verification hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): rotation hypotheses scored per second x pairs.
 Workload at any N: BASELINE config 2 per GPU — CO3D shape, B=32 pairs, 50 000
@@ -41,6 +41,7 @@ METRIC, UNIT = "rotation hypotheses scored/sec (x pairs)", "hyp*pairs/s"
 GATHER_BYTES_PER_HYP = 512 * 8 * 16 * 4      # SURVEY.md §8d: 262 144 B of smem gather per hypothesis (fp32)
 FLOP_PER_HYP = 1_843_200                     # SURVEY.md §8d
 HBM_BYTES_PER_HYP = 40                       # 36 B rotation in + 4 B score out
+DUMP_LIMIT_BYTES = 64_000_000                # --dump-outputs writes at most this much
 
 
 def load_peaks():
@@ -131,7 +132,8 @@ def synthetic_inputs(torch, pairs, hyps, seed=0):
 
 def cpu_reference_rate(torch, sample_pairs, sample_hyps, steps=1, warmup=0):
     """The reference's PyTorch CPU path (restated in oracle/ahv_oracle.py with the
-    same ATen calls) on all host threads, on a bounded sample of the workload."""
+    same ATen calls) on all host threads, on a bounded sample of the workload.  Also returns what the last step
+    computed, named as the product arm's outputs, plus the scores."""
     from oracle import ahv_oracle as orc
 
     cores = os.cpu_count() or 1
@@ -143,16 +145,18 @@ def cpu_reference_rate(torch, sample_pairs, sample_hyps, steps=1, warmup=0):
         t0 = time.perf_counter()
         s = orc.score_torch(vs, vt, R, W1, W2, b2)
         best = torch.max(s, dim=1)
-        _ = R[best.indices]
+        R_best = R[best.indices]
         dt = time.perf_counter() - t0
         if i >= warmup:
             times.append(dt)
     per_step = sum(times) / len(times)
+    last = {"topk_val": best.values[:, None].float(), "topk_idx": best.indices[:, None].double(),
+            "R_best": R_best[:, None].float(), "scores": s.float()}
     return {"value": sample_pairs * sample_hyps / per_step, "unit": UNIT, "cores": cores, "kind": "port",
             "threads": torch.get_num_threads(),
             "sample": f"{sample_pairs} pairs x {sample_hyps} hypotheses of the config-2 workload, "
                       f"oracle.score_torch (F.affine_grid/F.grid_sample/conv1x1/normalize, the reference's ATen calls), "
-                      f"{per_step:.2f} s per pass"}, per_step
+                      f"{per_step:.2f} s per pass"}, per_step, last
 
 
 def run_reference(args):
@@ -162,7 +166,9 @@ def run_reference(args):
     if rank != 0:
         return
     sp, sh = 2, 10000
-    base, per_step = cpu_reference_rate(torch, sp, sh, steps=max(1, args.steps), warmup=min(args.warmup, 1))
+    base, per_step, last = cpu_reference_rate(torch, sp, sh, steps=max(1, args.steps), warmup=min(args.warmup, 1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     line = {"impl": "reference", "metric": METRIC, "value": base["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": args.steps, "warmup": min(args.warmup, 1), "ms_per_step": per_step * 1e3, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -179,6 +185,25 @@ def run_reference(args):
 
 def _events(torch, n):
     return [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(n)]
+
+
+def dump_outputs(out_dir, tensors, limit_bytes=DUMP_LIMIT_BYTES):
+    """Write each tensor as out_dir/<name>.npy, so that two builds run with the same arguments (hence the same seeded
+    inputs) can be compared output for output.  The tensors share their leading (pair) axis; when together they
+    exceed `limit_bytes`, a fixed seeded sample of pairs is written instead and its pair numbers go to rows.npy."""
+    import numpy as np
+
+    arrays = {name: t.cpu().numpy() for name, t in tensors.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > limit_bytes:
+        pairs = next(iter(arrays.values())).shape[0]
+        keep = max(1, (limit_bytes - 4096) * pairs // (total + 8 * pairs))    # 8 B for each row number, 4 KiB for headers
+        rows = np.sort(np.random.default_rng(0).choice(pairs, keep, replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def gpu_eager_rate(torch, dev, sample_pairs, sample_hyps):
@@ -250,18 +275,20 @@ def run_ours(args):
 
     def timed(step_fn, n_steps, n_warm):
         """W untimed steps, then K steps each bracketed by CUDA events on the launching stream with the L2 flushed
-        (untimed) in between; barrier + synchronize on both sides; MAX over ranks of the summed step times."""
+        (untimed) in between; barrier + synchronize on both sides.  Returns the MAX over ranks of the summed step
+        times and what the last timed step returned."""
+        out = None
         for _ in range(n_warm):
-            step_fn()
+            out = step_fn()
         barrier()
         ev = _events(torch, n_steps)
         for a, b_ in ev:
             flush.zero_()
             a.record()
-            step_fn()
+            out = step_fn()
             b_.record()
         barrier()
-        return max_over_ranks(sum(a.elapsed_time(b_) for a, b_ in ev))[0]
+        return max_over_ranks(sum(a.elapsed_time(b_) for a, b_ in ev))[0], out
 
     def make_step(verifier, vs, vt, R, B, N, shard_lo, k=1):
         ws = verifier._workspace(B, N, k, dev)
@@ -308,8 +335,10 @@ def run_ours(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    total_ms = timed(step, steps, warmup)
+    total_ms, last = timed(step, steps, warmup)
     n_launch = launches_per_step * steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"topk_val": last[0].float(), "topk_idx": last[1].double(), "R_best": last[2].float()})
 
     # ------------------------------------------------ sharded parity: the exchange's winners vs an unsharded recompute
     sharded_parity = None
@@ -391,7 +420,7 @@ def run_ours(args):
             svs, svt = svs_h.bfloat16().to(dev), svt_h.to(dev)
             sR = ahv.ops.rotations_from_normals(snorm[slo:shi].contiguous().to(dev))
             sstep, _ = make_step(sver, svs, svt, sR, sB, shi - slo, slo)
-            c3_ms = timed(sstep, steps, warmup) / steps
+            c3_ms = timed(sstep, steps, warmup)[0] / steps
             strong = {"config3": {"workload": f"BASELINE configs[2]: B={sB} pairs, bf16 volumes, ONE set of {sN} hypotheses sharded "
                                               f"over {world} GPU(s), top-1, exchange inside the scoring kernel",
                                   "ms_per_step": c3_ms, "value": sB * sN / (c3_ms * 1e-3), "unit": UNIT, "scaling": "strong"}}
@@ -583,7 +612,7 @@ def run_ours(args):
         if eager is not None:
             line["gpu_eager_baseline"] = eager
         if world == 1 and not args.no_cpu:
-            base, _ = cpu_reference_rate(torch, 2, 10000)
+            base, _, _ = cpu_reference_rate(torch, 2, 10000)
             line["cpu_baseline"] = base
         print(json.dumps(line), flush=True)
     if world > 1:
@@ -610,7 +639,12 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="skip the training_step sub-record (profiling runs: keeps the launch list to the path)")
     ap.add_argument("--config", type=int, choices=[2, 3], default=2,
                     help="2 (default): BASELINE configs[1], weak scaling; 3: configs[2], bf16 volumes, hypothesis set sharded (strong)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (topk_val, topk_idx, R_best; the reference arm also "
+                         "its scores) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

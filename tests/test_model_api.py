@@ -1,15 +1,12 @@
 """CPU: the drop-in model keeps the reference's API and state-dict names."""
-import importlib.util
 import json
 import os
-import sys
-import types
 
+import numpy as np
 import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 def test_feature_aligner_state_dict_matches_reference_names():
@@ -36,39 +33,24 @@ def test_forward_2d3d_shapes_and_determinism():
     assert torch.equal(s1, s2) and torch.equal(t1, t2)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
-def test_forward_2d3d_matches_reference_module():
-    """Same state dict -> same volumes as the reference's own Feature_Aligner."""
-    code = r'''
-import sys, types, importlib.util, torch
-for name in ("matplotlib", "matplotlib.pyplot", "pytorch3d", "pytorch3d.transforms"):
-    sys.modules.setdefault(name, types.ModuleType(name))
-sys.modules["matplotlib"].pyplot = sys.modules["matplotlib.pyplot"]
-sys.modules["pytorch3d.transforms"].matrix_to_rotation_6d = lambda x: x
-sys.path.insert(0, "/root/reference")
-from modules.modules import Feature_Aligner as Ref
-import modules.modules as rm
-assert rm.__file__.startswith("/root/reference")
-def load(name, path):
-    spec = importlib.util.spec_from_file_location(name, path); m = importlib.util.module_from_spec(spec)
-    sys.modules[name] = m; spec.loader.exec_module(m); return m
-mine_att = load("mine_att", ROOT + "/transformer/attention.py")
-saved = sys.modules["transformer.attention"]; sys.modules["transformer.attention"] = mine_att
-mine = load("mine_mod", ROOT + "/modules/modules.py"); sys.modules["transformer.attention"] = saved
-torch.manual_seed(0)
-ref = Ref(768, 256, 32, 4, 4).eval(); me = mine.Feature_Aligner(768, 256, 32, 4, 4).eval()
-me.load_state_dict(ref.state_dict(), strict=True)
-with torch.no_grad():
-    a, b = torch.randn(2, 768, 8, 8), torch.randn(2, 768, 8, 8)
-    r = ref.forward_2d3d(a, b, random_mask=False, mask_ratio=0.0); m = me.forward_2d3d(a, b, random_mask=False, mask_ratio=0.0)
-err = max((r[0] - m[0]).abs().max().item(), (r[1] - m[1]).abs().max().item())
-assert err < 5e-5, err
-print("OK", err)
-'''.replace("ROOT", repr(ROOT))
-    import subprocess
+def test_forward_2d3d_matches_reference_module(golden):
+    """Same initialisation -> same volumes as the reference's own Feature_Aligner.  oracle/make_golden.py built the
+    reference's Feature_Aligner(768, 256, 32, 4, 4) under seed 0, stored its head weights in weights.npz and the
+    volumes its forward_2d3d made from two seeded [3, 768, 8, 8] inputs in shared_n3000_b3.npz; the same recipe is
+    rerun here on this implementation."""
+    from modules.modules import Feature_Aligner
 
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
-    assert out.returncode == 0 and "OK" in out.stdout, out.stderr[-2000:]
+    torch.manual_seed(0)
+    fa = Feature_Aligner(in_channel=768, mid_channel=256, out_channel=32, n_heads=4, depth=4).eval()
+    sd, w = fa.state_dict(), golden["weights"]
+    assert np.array_equal(sd["feature_embedding_2d.0.weight"].reshape(32, 384).numpy(), w["W1"])
+    assert np.array_equal(sd["feature_embedding_2d.2.weight"].reshape(32, 32).numpy(), w["W2"])
+    assert np.array_equal(sd["feature_embedding_2d.2.bias"].numpy(), w["b2"])
+    with torch.no_grad():
+        src, tgt = fa.forward_2d3d(torch.randn(3, 768, 8, 8), torch.randn(3, 768, 8, 8), random_mask=False, mask_ratio=0.0)
+    g = golden["shared_n3000_b3"]
+    err = max(float(np.abs(src.numpy() - g["vol_src"]).max()), float(np.abs(tgt.numpy() - g["vol_tgt"]).max()))
+    assert err < 5e-5, err
 
 
 class _TinyBackbone(torch.nn.Module):
@@ -172,3 +154,4 @@ def test_reference_shaped_checkpoint_loads():
             c = loaded(img, img.flip(-1))
         assert torch.allclose(a[0], c[0], atol=1e-5)
         assert Estimator.load_from_checkpoint(path).num_rota == _cfg()["DATA"]["NUM_ROTA"]    # cfg from hyper_parameters
+
