@@ -33,6 +33,8 @@ SIGNATURES = {
     "ahv_resblock3d": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _vp]),
     "ahv_score_train": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _vp, _sz, _vp]),
     "ahv_score_backward_saved": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _vp]),
+    "ahv_rotate_volume_grad_R": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i64, _vp]),
+    "ahv_score_backward_ex": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _vp]),
     "ahv_forward_3d2d": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _vp]),
     "ahv_workspace_bytes": (_sz, [_i, _i64, _i]),
     "ahv_score": (_i, [_vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _i64, _i, _vp, _sz, _vp]),

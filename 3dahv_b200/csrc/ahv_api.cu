@@ -99,6 +99,30 @@ AHV_API int ahv_score_backward(const float* vol_src, const float* tgt_feat, cons
                           grad_W1, grad_W2, grad_b2, B, N, (cudaStream_t)stream);
 }
 
+AHV_API int ahv_rotate_volume_grad_R(const float* vol, int vol_per_rotation, const float* R, const float* base,
+                                     const float* grad_out, float* grad_R, int64_t n, void* stream) {
+  if (n < 0 || (n > 0 && (!vol || !R || !base || !grad_out || !grad_R))) return AHV_EINVAL;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  return launch_rotate_volume_grad_R(vol, vol_per_rotation != 0, R, base, grad_out, grad_R, n, (cudaStream_t)stream);
+}
+
+AHV_API int ahv_score_backward_ex(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
+                                  const float* W1, const float* W2, const float* b2, const float* base,
+                                  const float* grad_scores, const void* h1_saved, const float* pair_inv_scale,
+                                  float* grad_vol, float* grad_tgt, float* grad_W1, float* grad_W2, float* grad_b2,
+                                  float* grad_R, int B, int64_t N, void* stream) {
+  if (B < 0 || N < 0 || N > 0x7fffffffLL) return AHV_EINVAL;
+  if (!grad_vol && !grad_tgt && !grad_W1 && !grad_W2 && !grad_b2 && !grad_R) return AHV_EINVAL;
+  if (!h1_saved != !pair_inv_scale || !aligned16(h1_saved)) return AHV_EINVAL;
+  if ((int64_t)B * N > 0 && (!vol_src || !tgt_feat || !R || !W1 || !W2 || !b2 || !base || !grad_scores))
+    return AHV_EINVAL;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  return launch_score_bwd(vol_src, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, grad_scores, grad_vol, grad_tgt,
+                          grad_W1, grad_W2, grad_b2, B, N, (cudaStream_t)stream, h1_saved, pair_inv_scale, grad_R);
+}
+
 AHV_API int ahv_infonce(const float* scores, const float* R, int r_per_pair, const float* gt_R, float acc_thr_deg,
                         float temperature, float* loss, float* grad_scores, int B, int64_t N, void* stream) {
   if (B < 0 || N < 1 || !(temperature > 0.0f)) return AHV_EINVAL;

@@ -48,15 +48,20 @@ struct Tap {
 
 __device__ __forceinline__ float unnorm(float g) { return fmaf(__fadd_rn(g, 1.0f), 4.0f, -0.5f); }
 
-__device__ __forceinline__ Tap make_tap(const float* R, float x, float y, float z) {
-  // grid = R @ (x, y, z); x -> W, y -> H, z -> D
-  float gx = fmaf(R[2], z, fmaf(R[1], y, R[0] * x));
-  float gy = fmaf(R[5], z, fmaf(R[4], y, R[3] * x));
-  float gz = fmaf(R[8], z, fmaf(R[7], y, R[6] * x));
+// Un-normalised, unclamped sample position (ix, iy, iz) of base point (x, y, z): grid = R @ (x, y, z);
+// x -> W, y -> H, z -> D
+__device__ __forceinline__ float3 sample_coords(const float* R, float x, float y, float z) {
+  const float gx = fmaf(R[2], z, fmaf(R[1], y, R[0] * x));
+  const float gy = fmaf(R[5], z, fmaf(R[4], y, R[3] * x));
+  const float gz = fmaf(R[8], z, fmaf(R[7], y, R[6] * x));
+  return make_float3(unnorm(gx), unnorm(gy), unnorm(gz));
+}
+
+__device__ __forceinline__ Tap tap_at(float3 u) {
   // clamp to [-1, 8]: anything outside only ever touches the zero halo
-  float ix = fminf(fmaxf(unnorm(gx), -1.0f), 8.0f);
-  float iy = fminf(fmaxf(unnorm(gy), -1.0f), 8.0f);
-  float iz = fminf(fmaxf(unnorm(gz), -1.0f), 8.0f);
+  float ix = fminf(fmaxf(u.x, -1.0f), 8.0f);
+  float iy = fminf(fmaxf(u.y, -1.0f), 8.0f);
+  float iz = fminf(fmaxf(u.z, -1.0f), 8.0f);
   float x0 = fminf(floorf(ix), 7.0f), y0 = fminf(floorf(iy), 7.0f), z0 = fminf(floorf(iz), 7.0f);
   Tap t;
   t.fx = ix - x0;
@@ -64,6 +69,10 @@ __device__ __forceinline__ Tap make_tap(const float* R, float x, float y, float 
   t.fz = iz - z0;
   t.line = (((int)z0 + 1) * kHalo + ((int)y0 + 1)) * kHalo + ((int)x0 + 1);
   return t;
+}
+
+__device__ __forceinline__ Tap make_tap(const float* R, float x, float y, float z) {
+  return tap_at(sample_coords(R, x, y, z));
 }
 
 // (score, index) -> one ordered 64-bit key: larger key = higher score, ties -> lower index
@@ -94,11 +103,13 @@ int launch_rotate_volume(const float* vol, int per_rot, const float* R, const fl
                          float* out, int64_t n, cudaStream_t s);
 int launch_rotate_volume_bwd(const float* grad_out, int per_rot, const float* R, const float* base,
                              float* grad_vol, int64_t n, cudaStream_t s);
+int launch_rotate_volume_grad_R(const float* vol, int per_rot, const float* R, const float* base, const float* grad_out,
+                                float* grad_R, int64_t n, cudaStream_t s);
 int launch_score_bwd(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
                      const float* W1, const float* W2, const float* b2, const float* base,
                      const float* grad_scores, float* g_vol, float* g_tgt, float* g_W1, float* g_W2,
                      float* g_b2, int B, int64_t N, cudaStream_t s, const void* h1_saved = nullptr,
-                     const float* pair_inv = nullptr);
+                     const float* pair_inv = nullptr, float* g_R = nullptr);
 int launch_score_bwd_tc(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
                         const float* W1, const float* W2, const float* b2, const float* base,
                         const float* grad_scores, const void* h1_saved, const float* pair_inv, float* g_vol,

@@ -175,6 +175,56 @@ __device__ __forceinline__ void conv2_bias(const Fp32Smem& sm, const float* b2r,
   }
 }
 
+// ---- rotation gradient of the trilinear resampling (utils.py:113-131 differentiated in its grid) -----------
+// Output voxel X[c] = trilinear(V[c], i) at i = (ix, iy, iz) = 4 (R b) + 3.5 (sample_coords), b = (base[w], base[h],
+// base[d]).  Given the upstream gradient gx4 = dL/dX[4j .. 4j+3] this adds sum_c dL/dX[c] dX[c]/di (x) b to G (3x3,
+// row-major); dL/dR = 4 G once summed over voxels and channel quads.  ATen's grid_sampler_3d_backward convention: the
+// corner is floor(i) (forward difference at an exact integer), a tap outside the volume reads the zero halo, and the
+// derivative along an axis is zero unless -1 <= i < 8 on that axis, tested on the unclamped coordinate (tap_at clamps
+// to [-1, 8] and caps the corner at 7, which would otherwise turn it into -V[7] or V[0]).  `vol` is the halo'd
+// shared-memory volume of stage_volume.
+__device__ __forceinline__ void rot_grad_accum(const float* vol, const float* R, float bx, float by, float bz, int j,
+                                               float4 gx4, float (&G)[9]) {
+  const float3 u = sample_coords(R, bx, by, bz);
+  const Tap t = tap_at(u);
+  const float* p = vol + t.line * kC + j * 4;
+  float dx = 0.0f, dy = 0.0f, dz = 0.0f;
+#pragma unroll
+  for (int k = 0; k < 8; ++k) {  // corner (ex, ey, ez) = (k & 1, (k >> 1) & 1, k >> 2)
+    const int ex = k & 1, ey = (k >> 1) & 1, ez = k >> 2;
+    const float4 a = *reinterpret_cast<const float4*>(p + (ez * kHalo * kHalo + ey * kHalo + ex) * kC);
+    const float cv = fmaf(gx4.w, a.w, fmaf(gx4.z, a.z, fmaf(gx4.y, a.y, gx4.x * a.x)));   // <dL/dX, V[corner]>
+    const float wx = ex ? t.fx : 1.0f - t.fx, wy = ey ? t.fy : 1.0f - t.fy, wz = ez ? t.fz : 1.0f - t.fz;
+    dx = fmaf(ex ? cv : -cv, wy * wz, dx);
+    dy = fmaf(ey ? cv : -cv, wx * wz, dy);
+    dz = fmaf(ez ? cv : -cv, wx * wy, dz);
+  }
+  dx = (u.x >= -1.0f && u.x < 8.0f) ? dx : 0.0f;
+  dy = (u.y >= -1.0f && u.y < 8.0f) ? dy : 0.0f;
+  dz = (u.z >= -1.0f && u.z < 8.0f) ? dz : 0.0f;
+  G[0] = fmaf(dx, bx, G[0]); G[1] = fmaf(dx, by, G[1]); G[2] = fmaf(dx, bz, G[2]);
+  G[3] = fmaf(dy, bx, G[3]); G[4] = fmaf(dy, by, G[4]); G[5] = fmaf(dy, bz, G[5]);
+  G[6] = fmaf(dz, bx, G[6]); G[7] = fmaf(dz, by, G[7]); G[8] = fmaf(dz, bz, G[8]);
+}
+
+// CTA-wide sum of the 9 accumulators, times `scale`, returned in threads 0..8 (element threadIdx.x); red: 72 floats of
+// shared memory.  One __syncthreads; the caller synchronises before red is written again.
+__device__ __forceinline__ float block_sum9(float (&G)[9], float* red, float scale) {
+#pragma unroll
+  for (int e = 0; e < 9; ++e) G[e] = warp_sum(G[e]);
+  if ((threadIdx.x & 31) == 0) {
+#pragma unroll
+    for (int e = 0; e < 9; ++e) red[(threadIdx.x >> 5) * 9 + e] = G[e];
+  }
+  __syncthreads();
+  float s = 0.0f;
+  if (threadIdx.x < 9) {
+#pragma unroll
+    for (int w = 0; w < kThreads / 32; ++w) s += red[w * 9 + threadIdx.x];
+  }
+  return s * scale;
+}
+
 __device__ __forceinline__ float quad_sum(float x) {
   x += __shfl_xor_sync(0xffffffffu, x, 1);
   x += __shfl_xor_sync(0xffffffffu, x, 2);

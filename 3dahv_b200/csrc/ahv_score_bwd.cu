@@ -12,6 +12,8 @@
 //                                    dH1 = (dH2 W2) * [H1 > 0];   dW1 += dH1^T A;   dA = dH1 W1
 //                                    dX = fold(dA)  (three views onto the rotated volume)
 //                                    dV_b += rotate^T(dX, R_n)   (adjoint of the trilinear resampling)
+//                                    dR_n += 4 sum_v (sum_c dX[c,v] dX[c,v]/di) b_v^T   (ahv_score_backward_ex only:
+//                                    the resampling differentiated in its grid, i = 4 R b + 3.5; DESIGN.md §4.4)
 //
 // fp32 FFMA throughout (gradients match fp64 autograd of the oracle to ~1e-6 of their maximum).
 // One CTA = 256 threads, 1 CTA / SM, contiguous range of (pair, hypothesis) items.  Persistent
@@ -45,6 +47,8 @@ static_assert(offsetof(Fp32Smem, rotT) == offsetof(Fp32Smem, rotA) + sizeof(floa
               offsetof(Fp32Smem, h1s) == offsetof(Fp32Smem, rotT) + sizeof(float) * kC * kRotC, "rotA, rotT, h1s are contiguous");
 static_assert((kDxFloats + 2 * kVox * 8) <= 2 * kC * kRotC + kP * kH1Row, "dX and the work list fit the dead buffers");
 static_assert(2 * kVox * sizeof(int) <= sizeof(float) * kP * kH1Row, "counters fit the dH2 buffer");
+static_assert((2 * kVox + 9 * kThreads / 32) * sizeof(float) <= sizeof(float) * kP * kH1Row,
+              "the rotation phase's partial sums fit behind the counters");
 
 // output voxel (z*64 + y*8 + x) a thread lists for the adjoint: lane bits -> x2 x1 y2 y1 z2, warp bits and j -> the rest
 __device__ __forceinline__ int adjoint_out_voxel(int t, int j) {
@@ -53,13 +57,17 @@ __device__ __forceinline__ int adjoint_out_voxel(int t, int j) {
   return z * 64 + y * 8 + x;
 }
 
+// kEx (ahv_score_backward_ex): every gradient output may be NULL - its accumulation and, for g_vol / g_W1 / g_R, its
+// phase are skipped - and the rotation-gradient phase (dS/dR into g_R) is compiled in.  kEx = false is the plain
+// backward of ahv_score_backward / ahv_score_backward_saved, which writes all five.
+template <bool kEx>
 __global__ void __launch_bounds__(kThreads, 1)
 score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tgt_feat,
                  const float* __restrict__ R, int r_per_pair, const float* __restrict__ W1,
                  const float* __restrict__ W2, const float* __restrict__ b2, const float* __restrict__ base,
                  const float* __restrict__ grad_scores, float* __restrict__ g_vol, float* __restrict__ g_tgt,
                  float* __restrict__ g_W1, float* __restrict__ g_W2, float* __restrict__ g_b2, int B, int64_t N,
-                 const __half* __restrict__ h1_saved, const float* __restrict__ pair_inv) {
+                 const __half* __restrict__ h1_saved, const float* __restrict__ pair_inv, float* __restrict__ g_R) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   BwdSmem& bs = *reinterpret_cast<BwdSmem*>(smem_raw);
   Fp32Smem& sm = bs.f;
@@ -67,6 +75,8 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
   const int64_t lo = total * blockIdx.x / gridDim.x, hi = total * (blockIdx.x + 1) / gridDim.x;
   if (lo >= hi) return;
   const int t = threadIdx.x;
+  const bool want_vol = !kEx || g_vol, want_tgt = !kEx || g_tgt, want_W1 = !kEx || g_W1;
+  const bool want_W2 = !kEx || g_W2, want_b2 = !kEx || g_b2, want_R = kEx && g_R;
   stage_weights(sm, W1, W2, base);
   // conv2 / normalise mapping: thread = (position, 8 output channels cg2*8 ..)
   const int pos = t >> 2, cg2 = t & 3;
@@ -95,14 +105,14 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
   auto flush_pair = [&](int b) {  // dT and dV of pair b leave the CTA
 #pragma unroll
     for (int oo = 0; oo < 8; ++oo) {
-      if (aT[oo] != 0.0f) atomicAdd(g_tgt + ((size_t)b * kO + cg2 * 8 + oo) * kP + pos, aT[oo]);
+      if (want_tgt && aT[oo] != 0.0f) atomicAdd(g_tgt + ((size_t)b * kO + cg2 * 8 + oo) * kP + pos, aT[oo]);
       aT[oo] = 0.0f;
     }
 #pragma unroll
     for (int j = 0; j < 2; ++j)
 #pragma unroll
       for (int c = 0; c < kC; ++c) {
-        if (aV[j][c] != 0.0f) atomicAdd(g_vol + ((size_t)b * kC + c) * kVox + t + 256 * j, aV[j][c]);
+        if (want_vol && aV[j][c] != 0.0f) atomicAdd(g_vol + ((size_t)b * kC + c) * kVox + t + 256 * j, aV[j][c]);
         aV[j][c] = 0.0f;
       }
   };
@@ -212,7 +222,7 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
     __syncthreads();
 
     // ---------------- dW1 += dH1^T A  (A = tri-plane views of the rotated volume) ----------------
-    {
+    if (want_W1) {
       const int cg = t & 15, c = t >> 4;
 #pragma unroll 1
       for (int pq = 0; pq < 16; ++pq) {
@@ -280,6 +290,28 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
       }
     }
 
+    // ---------------- dS/dR: the resampling differentiated in its grid (rot_grad_accum) ----------------
+    // dX (rotA, voxel-major, channels innermost), the halo'd source volume (sm.vol) and R (sm.Rcur, read from shared
+    // memory because the kernel runs at the register limit) are all in place.  Mapping of gather_hypothesis: 4 lanes
+    // per output voxel, 4 channels each.  The 9 partial sums meet in the dead dH2 buffer behind the adjoint's counters.
+    if (want_R) {
+      float G[9];
+#pragma unroll
+      for (int e = 0; e < 9; ++e) G[e] = 0.0f;
+      const int lane = t & 31, warp = t >> 5, j = lane & 3, w = lane >> 2;
+#pragma unroll 1
+      for (int pass = 0; pass < 8; ++pass) {
+        const int s = pass * 8 + warp, d = s >> 3, h = s & 7;
+        const float4 gx4 = *reinterpret_cast<const float4*>(sm.rotA + d * kDxD + h * kDxH + w * kDxW + 4 * j);
+        rot_grad_accum(sm.vol, sm.Rcur, sm.base[w], sm.base[h], sm.base[d], j, gx4, G);
+      }
+      const float sR = block_sum9(G, bs.dh2 + 2 * kVox, 4.0f);
+      if (t < 9) {
+        if (r_per_pair) g_R[(size_t)it * 9 + t] += sR;   // the item is this CTA's alone
+        else atomicAdd(g_R + (size_t)n * 9 + t, sR);
+      }
+    }
+
     // ---------------- dV_b += rotate^T(dX): adjoint of utils.py:113-131 as a gather ----------------
     // Output voxel vo feeds the 8 input voxels of its tap, corner(vo) + {0,1}^3, with the forward's weights.  Turned round:
     // every INPUT voxel gets the list of its (vo, weight) contributions - a counting sort over the <= 4096 contributions
@@ -287,7 +319,7 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
     // sums, 8-byte entries behind dX in the dead rotated-volume / dH1 buffers) - and the adjoint is one flat loop per
     // input voxel: exactly the contributing voxels, no geometry test, valid for any matrix R, fp32 weights recomputed from
     // the taps the forward gather recorded.
-    {
+    if (want_vol) {
       int* cnt = reinterpret_cast<int*>(bs.dh2);   // [512] contributions per input voxel
       int* start = cnt + kVox;                     // [512] exclusive prefix sum
       uint2* ent = reinterpret_cast<uint2*>(smem_raw + offsetof(BwdSmem, f) + offsetof(Fp32Smem, rotA) + sizeof(float) * kDxFloats);   // [<= 4096] (offset of dX[vo], weight), behind dX
@@ -383,19 +415,22 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
 #pragma unroll
       for (int kk = 0; kk < 8; ++kk) {
         const int k = view * 128 + c * 8 + kk;
-        atomicAdd(g_W1 + (2 * cg) * kK + k, aW1[view][kk][0]);
-        atomicAdd(g_W1 + (2 * cg + 1) * kK + k, aW1[view][kk][1]);
+        if (want_W1) {
+          atomicAdd(g_W1 + (2 * cg) * kK + k, aW1[view][kk][0]);
+          atomicAdd(g_W1 + (2 * cg + 1) * kK + k, aW1[view][kk][1]);
+        }
       }
     const int o = t >> 3, i0 = (t & 7) * 4;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) atomicAdd(g_W2 + o * kO + i0 + i, aW2[i]);
+    for (int i = 0; i < 4; ++i)
+      if (want_W2) atomicAdd(g_W2 + o * kO + i0 + i, aW2[i]);
     // db2: sum over the 64 positions inside the CTA first (threads with equal cg2 = t & 3)
     __syncthreads();
     float* red = sm.h1s;  // [4 cg2][8 oo][64 pos]
 #pragma unroll
     for (int oo = 0; oo < 8; ++oo) red[(cg2 * 8 + oo) * kP + pos] = ab2[oo];
     __syncthreads();
-    if (t < kO) {
+    if (want_b2 && t < kO) {
       float s = 0.0f;
       for (int p = 0; p < kP; ++p) s += red[t * kP + p];
       atomicAdd(g_b2 + t, s);
@@ -406,7 +441,8 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
 int launch_score_bwd(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
                      const float* W1, const float* W2, const float* b2, const float* base,
                      const float* grad_scores, float* g_vol, float* g_tgt, float* g_W1, float* g_W2,
-                     float* g_b2, int B, int64_t N, cudaStream_t s, const void* h1_saved, const float* pair_inv) {
+                     float* g_b2, int B, int64_t N, cudaStream_t s, const void* h1_saved, const float* pair_inv,
+                     float* g_R) {
   const int64_t total = (int64_t)B * N;
   if (total == 0) return AHV_OK;
   int dev = 0, sms = 0;
@@ -414,10 +450,16 @@ int launch_score_bwd(const float* vol_src, const float* tgt_feat, const float* R
   AHV_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   const unsigned grid = (unsigned)(total < sms ? total : sms);
   const size_t smem = sizeof(BwdSmem);
-  AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  score_bwd_kernel<<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
-                                                g_vol, g_tgt, g_W1, g_W2, g_b2, B, N,
-                                                static_cast<const __half*>(h1_saved), pair_inv);
+  const __half* h1 = static_cast<const __half*>(h1_saved);
+  if (g_R || !g_vol || !g_tgt || !g_W1 || !g_W2 || !g_b2) {
+    AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    score_bwd_kernel<true><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
+                                                        g_vol, g_tgt, g_W1, g_W2, g_b2, B, N, h1, pair_inv, g_R);
+  } else {
+    AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    score_bwd_kernel<false><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
+                                                         g_vol, g_tgt, g_W1, g_W2, g_b2, B, N, h1, pair_inv, nullptr);
+  }
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }

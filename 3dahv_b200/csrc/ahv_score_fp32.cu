@@ -7,6 +7,8 @@
 //  * forward_3d2d_kernel — modules/modules.py:112-124 on plain volumes
 //    (target features, refcompat).
 //  * rotate_volume_kernel — utils.py:113-131 materialised (refcompat only).
+//  * rotate_volume_bwd_kernel / rotate_volume_grad_R_kernel — its gradients w.r.t. the volume and the
+//    rotation (training variant, refcompat under autograd).
 //
 // Data layout in shared memory (one CTA = 256 threads, 1 CTA / SM):
 //   vol   [1000 lines][16 ch] fp32, zero halo          64000 B
@@ -214,6 +216,61 @@ int launch_rotate_volume_bwd(const float* grad_out, int per_rot, const float* R,
   const size_t smem = (kLines * kC + 8 + 12) * sizeof(float);
   AHV_CUDA_OK(cudaFuncSetAttribute(rotate_volume_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   rotate_volume_bwd_kernel<<<(unsigned)grid, kThreads, smem, s>>>(grad_out, per_rot, R, base, grad_vol, n, rpc);
+  AHV_CUDA_OK(cudaGetLastError());
+  return AHV_OK;
+}
+
+// ---- rotate_volume gradient with respect to the rotation ---------------------
+// grad_R[i] = dL/dR_i of out = rotate_volume(vol, R) given grad_out = dL/dout (rot_grad_accum, the same
+// formula as the fused backward's rotation phase).  The source volume is staged with its zero halo once per
+// CTA (shared) or once per rotation; one CTA handles `rot_per_cta` rotations and overwrites their grad_R.
+__global__ void __launch_bounds__(kThreads, 1)
+rotate_volume_grad_R_kernel(const float* __restrict__ vol, int per_rot, const float* __restrict__ R,
+                            const float* __restrict__ base, const float* __restrict__ grad_out,
+                            float* __restrict__ grad_R, int64_t n, int rot_per_cta) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  float* svol = reinterpret_cast<float*>(smem_raw);
+  float* sbase = svol + kLines * kC;
+  float* sR = sbase + 8;
+  float* red = sR + 12;  // [8 warps][9]
+  if (threadIdx.x < 8) sbase[threadIdx.x] = base[threadIdx.x];
+  const int64_t first = (int64_t)blockIdx.x * rot_per_cta;
+  for (int r = 0; r < rot_per_cta; ++r) {
+    const int64_t i = first + r;
+    if (i >= n) break;
+    if (per_rot || r == 0) {
+      __syncthreads();
+      stage_volume<float>(svol, vol + (per_rot ? (size_t)i * kC * kVox : 0));
+    }
+    __syncthreads();
+    if (threadIdx.x < 9) sR[threadIdx.x] = R[i * 9 + threadIdx.x];
+    __syncthreads();
+    float Rr[9];
+#pragma unroll
+    for (int e = 0; e < 9; ++e) Rr[e] = sR[e];
+    float G[9];
+#pragma unroll
+    for (int e = 0; e < 9; ++e) G[e] = 0.0f;
+    // task = (channel quad j, voxel v); consecutive lanes -> consecutive voxels (coalesced grad_out)
+    for (int task = threadIdx.x; task < 4 * kVox; task += kThreads) {
+      const int v = task & 511, j = task >> 9;
+      const int d = v >> 6, h = (v >> 3) & 7, w = v & 7;
+      const float* go = grad_out + ((size_t)i * kC + j * 4) * kVox + v;
+      rot_grad_accum(svol, Rr, sbase[w], sbase[h], sbase[d], j, make_float4(go[0], go[kVox], go[2 * kVox], go[3 * kVox]), G);
+    }
+    const float s = block_sum9(G, red, 4.0f);
+    if (threadIdx.x < 9) grad_R[i * 9 + threadIdx.x] = s;
+  }
+}
+
+int launch_rotate_volume_grad_R(const float* vol, int per_rot, const float* R, const float* base, const float* grad_out,
+                                float* grad_R, int64_t n, cudaStream_t s) {
+  if (n == 0) return AHV_OK;
+  const int rpc = per_rot ? 1 : 8;
+  const int64_t grid = (n + rpc - 1) / rpc;
+  const size_t smem = (kLines * kC + 8 + 12 + 72) * sizeof(float);
+  AHV_CUDA_OK(cudaFuncSetAttribute(rotate_volume_grad_R_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  rotate_volume_grad_R_kernel<<<(unsigned)grid, kThreads, smem, s>>>(vol, per_rot, R, base, grad_out, grad_R, n, rpc);
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }

@@ -125,6 +125,23 @@ def rotate_volume_backward(grad_out: torch.Tensor, R: torch.Tensor, per_rotation
     return out
 
 
+def rotate_volume_grad_R(vol: torch.Tensor, grad_out: torch.Tensor, R: torch.Tensor, per_rotation: bool) -> torch.Tensor:
+    """Gradient of rotate_volume w.r.t. the rotations, as F.grid_sample's backward gives it through F.affine_grid:
+    `vol` [16,8,8,8] (shared) or [n,16,8,8,8] (one per rotation), grad_out [n,16,8,8,8] -> grad_R [n,3,3]."""
+    v, g, R = _dev(vol, "vol"), _dev(grad_out, "grad_out"), _dev(R, "R")
+    n = R.shape[0]
+    if tuple(R.shape) != (n, 3, 3) or tuple(g.shape) != (n, 16, 8, 8, 8):
+        raise ValueError("R [n,3,3] and grad_out [n,16,8,8,8] expected")
+    if tuple(v.shape) != ((n, 16, 8, 8, 8) if per_rotation else (16, 8, 8, 8)):
+        raise ValueError("vol must be [n,16,8,8,8] (per rotation) or [16,8,8,8] (shared)")
+    out = torch.empty(n, 3, 3, device=g.device, dtype=torch.float32)
+    base = base_coords(g.device)
+    with torch.cuda.device(g.device):
+        _lib.check(_lib.lib().ahv_rotate_volume_grad_R(v.data_ptr(), int(per_rotation), R.data_ptr(), base.data_ptr(), g.data_ptr(),
+                                                       out.data_ptr(), n, _stream(g)), "ahv_rotate_volume_grad_R")
+    return out
+
+
 def score_train(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tensor, W1: torch.Tensor, W2: torch.Tensor,
                 b2: torch.Tensor, workspace: torch.Tensor | None = None):
     """ahv_score_train: the training forward - scores [B,N] from the tensor-core kernel, plus what the backward pass
@@ -152,14 +169,18 @@ def score_train(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tensor, 
     return scores, h1, pair_inv
 
 
-def score_backward(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tensor, W1: torch.Tensor, W2: torch.Tensor,
-                   b2: torch.Tensor, grad_scores: torch.Tensor, h1_saved: torch.Tensor | None = None,
-                   pair_inv: torch.Tensor | None = None, math: int = MATH_TC):
-    """Fused gradient of the verification scores (modules/model.py:53-56 under autograd): returns
-    (grad_vol_src [B,16,8,8,8], grad_tgt_feat [B,32,64], grad_W1 [32,384], grad_W2 [32,32], grad_b2 [32]).
-    With `h1_saved` / `pair_inv` from `score_train` the kernel reads conv1's output instead of recomputing it, and
-    `math` picks how it contracts dA = dH1 W1 and dW1 = dH1^T A: MATH_TC on tcgen05, MATH_FP32 in FFMA.  Without them
-    it is the exact fp32 kernel whatever `math` says."""
+def _score_backward_ex(vs, tg, R, W1, W2, b2, gs, h1, pi, outs, B, N, per_pair):
+    """ahv_score_backward_ex into `outs` = (grad_vol, grad_tgt, grad_W1, grad_W2, grad_b2, grad_R), each a zeroed
+    tensor or None."""
+    base = base_coords(vs.device)
+    ptr = lambda t: t.data_ptr() if t is not None else None
+    with torch.cuda.device(vs.device):
+        _lib.check(_lib.lib().ahv_score_backward_ex(vs.data_ptr(), tg.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(),
+                                                    W2.data_ptr(), b2.data_ptr(), base.data_ptr(), gs.data_ptr(), ptr(h1), ptr(pi),
+                                                    *(ptr(t) for t in outs), B, N, _stream(vs)), "ahv_score_backward_ex")
+
+
+def _score_backward_args(vol_src, tgt_feat, R, W1, W2, b2, grad_scores):
     vs, tg, R, gs = _dev(vol_src, "vol_src"), _dev(tgt_feat, "tgt_feat"), _dev(R, "R"), _dev(grad_scores, "grad_scores")
     W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
     B = vs.shape[0]
@@ -169,16 +190,37 @@ def score_backward(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tenso
         raise ValueError("vol_src [B,16,8,8,8], tgt_feat [B,32,64], grad_scores [B,N] expected")
     if per_pair and R.shape[0] != B:
         raise ValueError("per-pair rotations must be [B,N,3,3]")
+    return vs, tg, R, W1, W2, b2, gs, B, N, per_pair
+
+
+def score_backward(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tensor, W1: torch.Tensor, W2: torch.Tensor,
+                   b2: torch.Tensor, grad_scores: torch.Tensor, h1_saved: torch.Tensor | None = None,
+                   pair_inv: torch.Tensor | None = None, math: int = MATH_TC, want_grad_R: bool = False):
+    """Fused gradient of the verification scores (modules/model.py:53-56 under autograd): returns
+    (grad_vol_src [B,16,8,8,8], grad_tgt_feat [B,32,64], grad_W1 [32,384], grad_W2 [32,32], grad_b2 [32]).
+    With `h1_saved` / `pair_inv` from `score_train` the kernel reads conv1's output instead of recomputing it, and
+    `math` picks how it contracts dA = dH1 W1 and dW1 = dH1^T A: MATH_TC on tcgen05, MATH_FP32 in FFMA.  Without them
+    it is the exact fp32 kernel whatever `math` says.
+    `want_grad_R`: also the gradient w.r.t. the rotations, appended to the tuple - grad_R [N,3,3] (summed over pairs)
+    or [B,N,3,3] - from `ahv_score_backward_ex`, which contracts in fp32 FFMA whatever `math` says (the tcgen05
+    backward has no rotation phase; with saved activations this is the MATH_FP32 form on the same saved values)."""
+    vs, tg, R, W1, W2, b2, gs, B, N, per_pair = _score_backward_args(vol_src, tgt_feat, R, W1, W2, b2, grad_scores)
     dev = vs.device
     z = lambda *shape: torch.zeros(*shape, device=dev, dtype=torch.float32)
     g_vol, g_tgt, g_w1, g_w2, g_b2 = z(B, 16, 8, 8, 8), z(B, 32, 64), z(32, 384), z(32, 32), z(32)
+    h1 = pi = None
+    if h1_saved is not None:
+        h1 = _dev(h1_saved, "h1_saved", torch.float16)
+        pi = _dev(pair_inv, "pair_inv")
+        if h1.numel() != B * N * 64 * 32 or pi.numel() != B:
+            raise ValueError("h1_saved [B*N,64,32] fp16 and pair_inv [B] expected")
+    if want_grad_R:
+        g_R = z(*R.shape)
+        _score_backward_ex(vs, tg, R, W1, W2, b2, gs, h1, pi, (g_vol, g_tgt, g_w1, g_w2, g_b2, g_R), B, N, per_pair)
+        return g_vol, g_tgt, g_w1, g_w2, g_b2, g_R
     base = base_coords(dev)
     with torch.cuda.device(dev):
-        if h1_saved is not None:
-            h1 = _dev(h1_saved, "h1_saved", torch.float16)
-            pi = _dev(pair_inv, "pair_inv")
-            if h1.numel() != B * N * 64 * 32 or pi.numel() != B:
-                raise ValueError("h1_saved [B*N,64,32] fp16 and pair_inv [B] expected")
+        if h1 is not None:
             _lib.check(_lib.lib().ahv_score_backward_saved(vs.data_ptr(), tg.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(),
                                                            W2.data_ptr(), b2.data_ptr(), base.data_ptr(), gs.data_ptr(),
                                                            h1.data_ptr(), pi.data_ptr(), g_vol.data_ptr(), g_tgt.data_ptr(),
@@ -190,6 +232,17 @@ def score_backward(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tenso
                                                      g_vol.data_ptr(), g_tgt.data_ptr(), g_w1.data_ptr(), g_w2.data_ptr(),
                                                      g_b2.data_ptr(), B, N, _stream(vs)), "ahv_score_backward")
     return g_vol, g_tgt, g_w1, g_w2, g_b2
+
+
+def score_grad_R(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tensor, W1: torch.Tensor, W2: torch.Tensor,
+                 b2: torch.Tensor, grad_scores: torch.Tensor) -> torch.Tensor:
+    """d(sum grad_scores * scores)/dR alone - `ahv_score_backward_ex` with every other output NULL, so the kernel
+    skips the adjoint of the resampling and the dW1 contraction.  R [N,3,3] -> [N,3,3] (summed over pairs) or
+    [B,N,3,3] -> [B,N,3,3]."""
+    vs, tg, R, W1, W2, b2, gs, B, N, per_pair = _score_backward_args(vol_src, tgt_feat, R, W1, W2, b2, grad_scores)
+    g_R = torch.zeros(*R.shape, device=vs.device, dtype=torch.float32)
+    _score_backward_ex(vs, tg, R, W1, W2, b2, gs, None, None, (None, None, None, None, None, g_R), B, N, per_pair)
+    return g_R
 
 
 def infonce(scores: torch.Tensor, sampled_R: torch.Tensor, gt_delta_R: torch.Tensor, acc_thr_deg: float,

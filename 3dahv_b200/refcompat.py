@@ -7,7 +7,8 @@
 
 All of them run on the GPU through lib3dahv_b200 and raise on CPU tensors.  `rotate_volume` and `forward_3d2d`
 stay differentiable when autograd is recording and their inputs require a gradient (the reference trains through
-them, modules/model.py:53-56); otherwise they are single kernels with no autograd graph.
+them, modules/model.py:53-56; `rotate_volume` in the volume and in the rotation matrix, as F.grid_sample is);
+otherwise they are single kernels with no autograd graph.
 """
 from __future__ import annotations
 
@@ -26,7 +27,8 @@ def rotate_volume(volume: torch.Tensor, rotation_matrix: torch.Tensor, padding_m
         raise ValueError("volume must be [N,16,8,8,8]")
     shared = volume.stride(0) == 0 or volume.shape[0] == 1
     v = volume[0].float() if shared else volume.float()
-    if torch.is_grad_enabled() and volume.requires_grad:   # the reference back-propagates through this call (modules/model.py:53)
+    # the reference back-propagates through this call (modules/model.py:53), to the volume and to the rotations
+    if torch.is_grad_enabled() and (volume.requires_grad or rotation_matrix.requires_grad):
         from . import training
         return training.rotate_volume(v, rotation_matrix.float())
     return ops.rotate_volume(v, rotation_matrix.float())

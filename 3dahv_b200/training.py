@@ -25,6 +25,12 @@ hypothesis - `ahv_score_train`), and the backward (`ahv_score_backward_saved`, c
 instead of recomputing conv1 and runs its five contractions (conv2, dH1, dW2, dA, dW1) on tcgen05: 8.7 ms against
 24.8 ms for the 12 x 9000 step.  Its gradient is that of the function the forward evaluated (the forward's ReLU
 mask), with fp16 operand rounding - see `verification_scores`.
+
+Rotation gradients: the reference's rotate_volume (F.affine_grid + F.grid_sample) is differentiable in the rotation
+matrix as well, and so are `rotate_volume` and `verification_scores` here - `R.requires_grad_()` gives `R.grad`, with
+ATen's convention at lattice points and at the volume's edge (DESIGN.md §4.4).  The fused backward then runs
+`ahv_score_backward_ex`, the fp32 kernel with a rotation phase added; nothing changes for an R that needs no gradient.
+`infonce_loss` keeps `sampled_R` as data: its positive mask is a step function of R.
 """
 from __future__ import annotations
 
@@ -38,22 +44,26 @@ from ._lib import MATH_FP32, MATH_TC
 
 
 class _RotateVolume(torch.autograd.Function):
-    """utils.rotate_volume (utils.py:113-131) with a gradient w.r.t. the volume (rotations are data)."""
+    """utils.rotate_volume (utils.py:113-131) with gradients w.r.t. the volume and the rotations (F.grid_sample's
+    backward through F.affine_grid: `ahv_rotate_volume_backward` and `ahv_rotate_volume_grad_R`)."""
 
     @staticmethod
     def forward(ctx, volume, R):
         ctx.per_rot = volume.dim() == 5
-        ctx.save_for_backward(R)
+        ctx.save_for_backward(R, volume.detach() if ctx.needs_input_grad[1] else None)
         return ops.rotate_volume(volume.detach(), R)
 
     @staticmethod
     def backward(ctx, grad_out):
-        (R,) = ctx.saved_tensors
-        return ops.rotate_volume_backward(grad_out.contiguous(), R, ctx.per_rot), None
+        R, volume = ctx.saved_tensors
+        g = grad_out.contiguous()
+        g_vol = ops.rotate_volume_backward(g, R, ctx.per_rot) if ctx.needs_input_grad[0] else None
+        g_R = ops.rotate_volume_grad_R(volume, g, R, ctx.per_rot) if ctx.needs_input_grad[1] else None
+        return g_vol, g_R
 
 
 def rotate_volume(volume: torch.Tensor, R: torch.Tensor) -> torch.Tensor:
-    """Differentiable (w.r.t. `volume`) GPU rotate_volume: [16,8,8,8] or [n,16,8,8,8] with R [n,3,3]."""
+    """Differentiable (w.r.t. `volume` and `R`) GPU rotate_volume: [16,8,8,8] or [n,16,8,8,8] with R [n,3,3]."""
     return _RotateVolume.apply(volume, R)
 
 
@@ -73,13 +83,14 @@ def head_torch(vol: torch.Tensor, W1, W2, b2) -> torch.Tensor:
 
 class _VerifyScores(torch.autograd.Function):
     """scores[b,n] of modules/model.py:53-56; forward fused, backward fused (exact fp32 kernel, saved-activation
-    tensor-core kernel) or chunked recomputation."""
+    tensor-core kernel) or chunked recomputation.  R's gradient, when it needs one, comes from the fp32 kernel's
+    rotation phase (`ahv_score_backward_ex`) or, chunked, through `_RotateVolume`."""
 
     @staticmethod
     def forward(ctx, vol_src, vol_tgt, R, W1, W2, b2, math, chunk, fused_backward, save_activations, tc_backward=True):
         tgt = ops.forward_3d2d(vol_tgt.detach().float(), W1.detach(), W2.detach(), b2.detach())
         h1 = pair_inv = None
-        needs_grad = any(t.requires_grad for t in (vol_src, vol_tgt, W1, W2, b2))
+        needs_grad = any(t.requires_grad for t in (vol_src, vol_tgt, R, W1, W2, b2))
         if save_activations and fused_backward and math == MATH_TC and needs_grad and vol_src.dtype == torch.float32:
             # tensor-core forward that keeps conv1's ReLU'd output (4 KB per item) for the backward kernel
             scores, h1, pair_inv = ops.score_train(vol_src.detach(), tgt, R, W1.detach(), W2.detach(), b2.detach())
@@ -98,40 +109,46 @@ class _VerifyScores(torch.autograd.Function):
         B = vol_src.shape[0]
         per_pair = R.dim() == 4
         N = R.shape[1] if per_pair else R.shape[0]
+        want_R = ctx.needs_input_grad[2]
         if ctx.fused_backward:
-            g_vs, g_tgt, g_w1, g_w2, g_b = ops.score_backward(vol_src.detach().float(), tgt_saved, R, W1.detach().float(),
-                                                              W2.detach().float(), b2.detach().float(),
-                                                              grad_scores.contiguous().float(), h1, pair_inv, ctx.bwd_math)
+            # with R's gradient: ahv_score_backward_ex, the same fp32 kernel (and, with saved activations, the same kept
+            # values and ReLU mask) plus its rotation phase - the tcgen05 backward has none
+            g = ops.score_backward(vol_src.detach().float(), tgt_saved, R.detach(), W1.detach().float(), W2.detach().float(),
+                                   b2.detach().float(), grad_scores.contiguous().float(), h1, pair_inv, ctx.bwd_math,
+                                   want_grad_R=want_R)
+            g_vs, g_tgt, g_w1, g_w2, g_b = g[:5]
             with torch.enable_grad():   # target side: B volumes through the differentiable head
                 vt = vol_tgt.detach().float().requires_grad_(True)
                 w1, w2, bb = (t.detach().float().requires_grad_(True) for t in (W1, W2, b2))
                 gt = torch.autograd.grad(head_torch(vt, w1, w2, bb), [vt, w1, w2, bb], grad_outputs=g_tgt)
-            return (g_vs, gt[0], None, (g_w1 + gt[1].reshape(32, 384)).reshape(W1.shape),
+            return (g_vs, gt[0], g[5] if want_R else None, (g_w1 + gt[1].reshape(32, 384)).reshape(W1.shape),
                     (g_w2 + gt[2].reshape(32, 32)).reshape(W2.shape), g_b + gt[3], None, None, None, None, None)
         with torch.enable_grad():
             vs = vol_src.detach().float().requires_grad_(True)
             vt = vol_tgt.detach().float().requires_grad_(True)
             w1, w2, bb = (t.detach().float().requires_grad_(True) for t in (W1, W2, b2))
+            Rl = R.detach().requires_grad_(want_R)
             tgt = head_torch(vt, w1, w2, bb)                                # [B,32,64]
             tgt_leaf = tgt.detach().requires_grad_(True)                    # cut here: tgt's own graph is walked once, below
             total = None
             for b in range(B):
-                Rb = R[b] if per_pair else R
+                Rb = Rl[b] if per_pair else Rl
                 for a in range(0, N, ctx.chunk):
                     Rc = Rb[a:a + ctx.chunk].contiguous()
                     f = head_torch(rotate_volume(vs[b], Rc), w1, w2, bb)   # recomputed, freed after this chunk
                     s = (f * tgt_leaf[b][None]).sum(dim=1).mean(dim=-1)
                     part = (s * grad_scores[b, a:a + ctx.chunk]).sum()
                     # backward per chunk keeps the live graph at chunk size
-                    gs = torch.autograd.grad(part, [vs, w1, w2, bb, tgt_leaf], allow_unused=True)
+                    gs = torch.autograd.grad(part, [vs, w1, w2, bb, tgt_leaf] + ([Rl] if want_R else []), allow_unused=True)
                     total = gs if total is None else tuple(x + y if (x is not None and y is not None) else (x if y is None else y)
                                                            for x, y in zip(total, gs))
-            g_vs, g_w1, g_w2, g_b, g_tgt = total
+            g_vs, g_w1, g_w2, g_b, g_tgt = total[:5]
+            g_R = total[5] if want_R else None
             # through the target features to vol_tgt and (again) the head weights
             gt = torch.autograd.grad(tgt, [vt, w1, w2, bb], grad_outputs=g_tgt, allow_unused=True)
             g_vt = gt[0]
             g_w1, g_w2, g_b = g_w1 + gt[1], g_w2 + gt[2], g_b + gt[3]
-        return g_vs, g_vt, None, g_w1.reshape(W1.shape), g_w2.reshape(W2.shape), g_b, None, None, None, None, None
+        return g_vs, g_vt, g_R, g_w1.reshape(W1.shape), g_w2.reshape(W2.shape), g_b, None, None, None, None, None
 
 
 def verification_scores(vol_src, vol_tgt, R, W1, W2, b2, math: int = MATH_TC, chunk: int = 1024,
@@ -147,7 +164,11 @@ def verification_scores(vol_src, vol_tgt, R, W1, W2, b2, math: int = MATH_TC, ch
     (measured 2.6 % of the maximum; tests/test_gpu_training.py).  The default recomputes and matches the reference's
     fp32 autograd to 1e-4.  With saved activations `tc_backward` (default) also moves the backward's two large
     contractions, dA = dH1 W1 and dW1 = dH1^T A, to tcgen05 with fp16 operands under power-of-two scales
-    (csrc/ahv_score_bwd_tc.cu); False keeps them in fp32 FFMA."""
+    (csrc/ahv_score_bwd_tc.cu); False keeps them in fp32 FFMA.
+    When `R` requires a gradient, `R.grad` is d/dR of the scores ([N,3,3] summed over pairs, or [B,N,3,3]).  The fused
+    backward computes it, and the other gradients, with `ahv_score_backward_ex` in fp32 FFMA; with saved activations
+    that call replaces the tcgen05 backward whatever `tc_backward` says (same kept values, same ReLU mask, fp32
+    contractions).  The chunked form differentiates through `rotate_volume` instead."""
     return _VerifyScores.apply(vol_src, vol_tgt, R.contiguous(), W1, W2, b2, math, chunk, fused_backward, save_activations,
                                tc_backward)
 

@@ -11,6 +11,7 @@ ever materialised).
 """
 from __future__ import annotations
 
+import math
 from dataclasses import dataclass
 
 import torch
@@ -109,6 +110,54 @@ class HypothesisVerifier:
                                                                   max_angle_deg=max_angle_deg, seed=seed, math=self.math,
                                                                   workspace=getattr(self, "_ws_refine", None))
         return bR, bv, VerifyResult(None, fv, fi, fR), cand
+
+    @torch.no_grad()
+    def refine_gradient(self, vol_src, vol_tgt, R_init, steps: int = 20, step_deg: float = 1.0):
+        """Gradient refinement of given rotations (extension): backtracking Riemannian gradient ascent of the
+        AHV_MATH_FP32 score on SO(3), every candidate at once.  R_init [B,3,3] or [B,k,3,3] (e.g. `VerifyResult.R_best`
+        of a top-k pass).  Each step takes G = dS/dR from the fused backward's rotation phase (`ops.score_grad_R`),
+        the tangent direction w_i = <G, [e_i]x R>, a trial rotation exp(theta [w/|w|]x) R, and keeps it only where it
+        scores higher (theta *= 1.2 there, /= 2 elsewhere).  Candidates are scored with the fp32 kernel from start to
+        end, so every returned score is >= its starting score.  A fixed number of steps, no host synchronisation:
+        CUDA-graph capturable.  Returns (R_best [B,3,3], score [B], R_all [B,k,3,3], score_all [B,k]); the best is
+        the per-pair arg-max over k, ties to the lowest index."""
+        dev = vol_src.device
+        W1, W2, b2 = self._weights_on(dev)
+        R = (R_init[:, None] if R_init.dim() == 3 else R_init).float().contiguous()
+        B, k = R.shape[:2]
+        vs = vol_src.float()
+        tgt = ops.forward_3d2d(vol_tgt.float(), W1, W2, b2)
+
+        def score(Rc):
+            return ops.score(vs, tgt, Rc, W1, W2, b2, k=0, math=MATH_FP32)[0]
+
+        s = score(R)
+        theta = torch.full((B, k), math.radians(step_deg), device=dev)
+        ones = torch.ones(B, k, device=dev)
+        eye = torch.eye(3, device=dev)
+        for _ in range(steps):
+            G = ops.score_grad_R(vs, tgt, R, W1, W2, b2, ones)
+            M = G @ R.transpose(-1, -2)                                    # <G, [e_i]x R> = <G R^T, [e_i]x>
+            w = torch.stack((M[..., 2, 1] - M[..., 1, 2], M[..., 0, 2] - M[..., 2, 0], M[..., 1, 0] - M[..., 0, 1]), -1)
+            u = w / w.norm(dim=-1, keepdim=True).clamp_min(1e-30)
+            K = _hat(u)
+            dR = eye + torch.sin(theta)[..., None, None] * K + (1.0 - torch.cos(theta))[..., None, None] * (K @ K)
+            Rt = dR @ R
+            Rt = 1.5 * Rt - 0.5 * Rt @ Rt.transpose(-1, -2) @ Rt           # one Newton step towards the nearest rotation
+            st = score(Rt)
+            acc = st > s
+            R = torch.where(acc[..., None, None], Rt, R).contiguous()
+            s = torch.where(acc, st, s)
+            theta = torch.where(acc, theta * 1.2, theta * 0.5)
+        best = torch.argmax(s, dim=1)                                      # first maximal index
+        rows = torch.arange(B, device=dev)
+        return R[rows, best], s[rows, best], R, s
+
+
+def _hat(u: torch.Tensor) -> torch.Tensor:
+    """[..., 3] -> the cross-product matrices [u]x [..., 3, 3]."""
+    z = torch.zeros_like(u[..., 0])
+    return torch.stack((z, -u[..., 2], u[..., 1], u[..., 2], z, -u[..., 0], -u[..., 1], u[..., 0], z), -1).reshape(*u.shape[:-1], 3, 3)
 
 
 class GraphedVerifier:

@@ -102,6 +102,13 @@ AHV_API int ahv_rotate_volume(const float* vol, int vol_per_rotation, const floa
 AHV_API int ahv_rotate_volume_backward(const float* grad_out, int vol_per_rotation, const float* R,
                                        const float* base, float* grad_vol, int64_t n, void* stream);
 
+/* dS/dR of ahv_rotate_volume (utils.py:113-131 differentiated in its grid, as F.grid_sample's backward does):
+ * grad_R [n,3,3] is overwritten.  vol as in ahv_rotate_volume, grad_out [n,16,8,8,8].  ATen's convention: corner =
+ * floor (forward difference at an exact integer coordinate), out-of-range taps contribute zero, and the derivative
+ * along an axis is zero unless -1 <= its un-normalised coordinate < 8. */
+AHV_API int ahv_rotate_volume_grad_R(const float* vol, int vol_per_rotation, const float* R, const float* base,
+                                     const float* grad_out, float* grad_R, int64_t n, void* stream);
+
 /* Gradient of the verification scores (training variant: the autograd path of modules/model.py:53-56 inside
  * infoNCE_loss, :43-63) in one fused kernel: for every (pair b, hypothesis n) the forward is recomputed in
  * shared memory and grad_scores[b,n] is pushed back to the source volume, the target features, W1, W2 and
@@ -139,6 +146,16 @@ AHV_API int ahv_score_backward_saved(const float* vol_src, const float* tgt_feat
                                      const float* grad_scores, const void* h1_saved, const float* pair_inv_scale,
                                      float* grad_vol, float* grad_tgt, float* grad_W1, float* grad_W2, float* grad_b2,
                                      int B, int64_t N, int math_mode, void* stream);
+/* ahv_score_backward / ahv_score_backward_saved plus the rotation gradient: h1_saved/pair_inv_scale both NULL =
+ * recompute conv1; each gradient output may be NULL (at least one not); grad_R [N,3,3] (summed over pairs) or
+ * [B,N,3,3], ADDED like the others.  fp32 FFMA in both forms (the saved-activation form is the AHV_MATH_FP32 kernel of
+ * ahv_score_backward_saved); the rotation gradient follows ahv_rotate_volume_grad_R's convention.  Outputs left NULL
+ * cost nothing: grad_R alone skips the adjoint of the resampling and the dW1 contraction. */
+AHV_API int ahv_score_backward_ex(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
+                                  const float* W1, const float* W2, const float* b2, const float* base,
+                                  const float* grad_scores, const void* h1_saved, const float* pair_inv_scale,
+                                  float* grad_vol, float* grad_tgt, float* grad_W1, float* grad_W2, float* grad_b2,
+                                  float* grad_R, int B, int64_t N, void* stream);
 
 /* infoNCE_loss given the scores (training variant, modules/model.py:43-63 / model_co3d.py:41-61), one launch:
  * positives of pair b = hypotheses whose rotation lies within acc_thr_deg of gt_R[b] (:46-49);
