@@ -55,7 +55,18 @@ enum { AHV_VOL_F32 = 0, AHV_VOL_BF16 = 1 };
  *                 HFMA2, halving the shared-memory gather traffic.  bf16 volumes always
  *                 take this path (their staging is exact).  About 2e-4 relative.
  * Normalisation, correlation and selection are fp32 in every mode; trilinear resampling is
- * fp32 except in the f16-gather path. */
+ * fp32 except in the f16-gather path.
+ * Dynamic range: the tensor-core modes multiply each pair's volume by a power of two that maps
+ * max|V| into (b/2, b], b = min(4096, 16384 / largest L1 row norm of W1), and undo it before the
+ * bias, so one large voxel pushes the rest of the volume towards fp16's subnormals.  Measured on an
+ * NVIDIA B200 (1000 W) against fp64, for a standard-normal volume with outlier voxels up to r times
+ * larger (scripts/dynamic_range.py, tests/test_gpu_pair_scale.py), the scores meet their gates as follows:
+ *   AHV_MATH_TC, fp32 volumes           1e-3 up to r = 1e8 (9.4e-4 there; 1.7e-2 at 1e9)
+ *   AHV_MATH_TC_F16GATHER, fp32 volumes 1e-3 up to r = 3e7 (7.4e-4 there; 1.5e-3 at 1e8)
+ *   bf16 volumes (either tensor-core mode) 2e-3 against the bf16-rounded volume and 1e-2 against the
+ *                                       unrounded one up to r = 1e8 (1.5e-3 there; 2.1e-2 at 1e9)
+ *   AHV_MATH_FP32                       2e-5 up to r = 3e5; beyond it fp32 rounding of the outlier's
+ *                                       share (the reference's fp32 path too) reaches 1e-4 at r = 1e7. */
 enum { AHV_MATH_TC = 0, AHV_MATH_FP32 = 1, AHV_MATH_TC_F16GATHER = 2 };
 
 AHV_API int ahv_version(void);

@@ -57,21 +57,23 @@ def _topk_or_tie(ref_scores, idx_gpu, tol):
 
 def test_config2_full_pairs_vs_oracle(ahv, golden, oracle):
     """configs[1]: CO3D, 32 pairs x the full 50 000-hypothesis set, fp32 volumes, one GPU.  Three WHOLE pairs
-    (150 000 hypothesis-pairs) against the oracle, the fused arg-max against the oracle's on those pairs."""
+    (150 000 hypothesis-pairs) against the oracle, the fused arg-max against the oracle's on those pairs; the same for
+    the opt-in AHV_MATH_TC_F16GATHER mode (fp16-staged volume), which is held to the same gate."""
     B, N = 32, 50000
     vs, vt = _volumes(B, 0)
     torch.manual_seed(0)
     R = ahv.so3.random_rotations(N, device=DEV)
-    v = _verifier(ahv, golden)
-    r = v.score(vs.to(DEV), vt.to(DEV), R, k=1, return_scores=True)
-    fused = v.score(vs.to(DEV), vt.to(DEV), R, k=1, return_scores=False)        # the 2-launch step bench.py times
-    assert torch.equal(fused.topk_idx, r.topk_idx) and torch.equal(fused.topk_val, r.topk_val)
-    assert torch.equal(fused.R_best[:, 0], R[fused.topk_idx[:, 0]])
     pairs = [0, 13, 31]
     ref = oracle.score_c(vs[pairs].numpy(), vt[pairs].numpy(), R.cpu().numpy(), *_weights(golden))
-    got = r.scores[pairs].cpu().numpy()
-    assert _relerr(got, ref) <= 1e-3
-    assert _top1_or_tie(ref, fused.topk_idx[pairs, 0].cpu().numpy(), 1e-3)
+    for math in (ahv.MATH_TC, ahv.MATH_TC_F16GATHER):
+        v = _verifier(ahv, golden, math)
+        r = v.score(vs.to(DEV), vt.to(DEV), R, k=1, return_scores=True)
+        fused = v.score(vs.to(DEV), vt.to(DEV), R, k=1, return_scores=False)    # the 2-launch step bench.py times
+        assert torch.equal(fused.topk_idx, r.topk_idx) and torch.equal(fused.topk_val, r.topk_val)
+        assert torch.equal(fused.R_best[:, 0], R[fused.topk_idx[:, 0]])
+        got = r.scores[pairs].cpu().numpy()
+        assert _relerr(got, ref) <= 1e-3, (math, _relerr(got, ref))
+        assert _top1_or_tie(ref, fused.topk_idx[pairs, 0].cpu().numpy(), 1e-3), math
 
 
 def test_config3_bf16_128_pairs_vs_oracle(ahv, golden, oracle):
