@@ -1,5 +1,6 @@
 // extern "C" surface of lib3dahv_b200 (see include/ahv_b200.h for the contract
 // and the reference interface each entry replaces).
+#include <cmath>
 #include <cstring>
 #include <new>
 
@@ -328,6 +329,72 @@ AHV_API int ahv_refine(const void* vol_src, int vol_dtype, const float* vol_tgt,
   // pass 2: per-pair candidate sets [B, k*m], arg-max
   return ahv_verify(vol_src, vol_dtype, vol_tgt, cand, 1, W1, W2, b2, base, nullptr, best_val, best_idx, R_best, 1, 0, B,
                     (int64_t)k * m, math_mode, ws + ws1, ws2, stream);
+}
+
+// ---- gradient ascent of the fp32 score on SO(3), alone and after the grid pass (extension) ---------------
+namespace {
+bool ascent_args_ok(int vol_dtype, int steps, float step_deg) {
+  return (vol_dtype == AHV_VOL_F32 || vol_dtype == AHV_VOL_BF16) && steps >= 0 && steps <= 1000 &&
+         std::isfinite(step_deg) && step_deg > 0.0f;   // the step cap bounds the runtime of one launch
+}
+}  // namespace
+
+AHV_API int ahv_gradient_ascent(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R_init,
+                                const float* W1, const float* W2, const float* b2, const float* base, int steps,
+                                float step_deg, float* R_out, float* score_out, int B, int K, void* stream) {
+  if (B < 1 || K < 1 || !ascent_args_ok(vol_dtype, steps, step_deg)) return AHV_EINVAL;
+  if (!vol_src || !tgt_feat || !R_init || !W1 || !W2 || !b2 || !base || !R_out || !score_out) return AHV_EINVAL;
+  if (!aligned16(vol_src) || !aligned16(tgt_feat) || !aligned16(R_init) || !aligned16(R_out) || !aligned16(W1) ||
+      !aligned16(W2))
+    return AHV_EINVAL;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  return launch_gradient_ascent(vol_src, vol_dtype, tgt_feat, R_init, W1, W2, b2, base, steps, step_deg, R_out, score_out,
+                                B, K, (cudaStream_t)stream);
+}
+
+// workspace = [ahv_verify's for the grid pass | target features B*32*64 fp32 | top-k partials over [B,k]]
+AHV_API size_t ahv_refine_gradient_workspace_bytes(int B, int64_t N, int k) {
+  if (B < 0 || N < 0 || k < 1 || k > kMaxK) return 0;
+  return ahv_workspace_bytes(B, N, k) + align_up((size_t)B * kO * kP * sizeof(float), 256) +
+         align_up(topk_workspace_bytes(B, k, 1), 256);
+}
+
+AHV_API int ahv_refine_gradient(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
+                                const float* W1, const float* W2, const float* b2, const float* base, int k, int steps,
+                                float step_deg, float* first_val, int64_t* first_idx, float* first_R, float* R_all,
+                                float* score_all, float* best_val, int64_t* best_idx, float* R_best, int B, int64_t N,
+                                int math_mode, void* workspace, size_t workspace_bytes, void* stream) {
+  if (B < 1 || N < 1 || N > 0x7fffffffLL || k < 1 || k > kMaxK || k > N) return AHV_EINVAL;
+  if (!ascent_args_ok(vol_dtype, steps, step_deg)) return AHV_EINVAL;
+  if (math_mode != AHV_MATH_TC && math_mode != AHV_MATH_FP32 && math_mode != AHV_MATH_TC_F16GATHER) return AHV_EINVAL;
+  if (!vol_src || !vol_tgt || !R || !W1 || !W2 || !b2 || !base || !first_val || !first_idx || !first_R || !R_all ||
+      !score_all || !best_val || !best_idx || !workspace)
+    return AHV_EINVAL;
+  if (!aligned16(vol_src) || !aligned16(vol_tgt) || !aligned16(R) || !aligned16(W1) || !aligned16(W2) ||
+      !aligned16(first_R) || !aligned16(R_all) || !aligned16(R_best) || !aligned16(workspace))
+    return AHV_EINVAL;
+  const size_t ws1 = ahv_workspace_bytes(B, N, k), ws_tgt = align_up((size_t)B * kO * kP * sizeof(float), 256);
+  const size_t ws_top = align_up(topk_workspace_bytes(B, k, 1), 256);
+  if (workspace_bytes < ws1 + ws_tgt + ws_top) return AHV_EWORKSPACE;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  cudaStream_t s = (cudaStream_t)stream;
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  float* tgt = reinterpret_cast<float*>(ws + ws1);
+  // pass 1: the whole set, top-k and their rotations
+  st = ahv_verify(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, first_val, first_idx, first_R, k, 0,
+                  B, N, math_mode, ws, ws1, stream);
+  if (st != AHV_OK) return st;
+  // the ascent scores in fp32 against fp32 target features (bit-equal to ahv_forward_3d2d), whatever math_mode is
+  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
+  if (st != AHV_OK) return st;
+  st = launch_gradient_ascent(vol_src, vol_dtype, tgt, first_R, W1, W2, b2, base, steps, step_deg, R_all, score_all, B, k, s);
+  if (st != AHV_OK) return st;
+  // per-pair arg-max over the k ascended candidates
+  st = launch_topk(score_all, B, k, 1, 0, best_val, best_idx, ws + ws1 + ws_tgt, ws_top, s);
+  if (st != AHV_OK || !R_best) return st;
+  return launch_gather_rotations(R_all, 1, best_idx, 0, B, k, 1, R_best, s);
 }
 
 // ---- hypothesis set sharded over the GPUs of one node: winners exchanged through peer memory -------------

@@ -121,6 +121,9 @@ int launch_resblock3d(const float* x, const float* Wc1, const float* Wc2, const 
                       cudaStream_t s);
 int launch_infonce(const float* scores, const float* R, int r_per_pair, const float* gt, float thr_deg, float temperature,
                    float* loss, float* grad, int B, int64_t N, cudaStream_t s);
+int launch_gradient_ascent(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R_init, const float* W1,
+                           const float* W2, const float* b2, const float* base, int steps, float step_deg, float* R_out,
+                           float* score_out, int B, int K, cudaStream_t s);
 int launch_forward_3d2d(const float* vol, const float* W1, const float* W2, const float* b2,
                         float* feat, int64_t m, cudaStream_t s);
 int launch_tgt_feat(const float* vol_tgt, const float* W1, const float* W2, const float* b2,

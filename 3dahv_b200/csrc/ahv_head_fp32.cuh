@@ -231,6 +231,34 @@ __device__ __forceinline__ float quad_sum(float x) {
   return x;
 }
 
+// ---- the score of one hypothesis: mean over the 64 positions of <F_p, T_p>, F = H2 / max(|H2|, 1e-12) --------
+// ss = |H2_p|^2 and dt = <H2_p, T_p> over the 32 channels of this thread's position (the 4 lanes of its quad), from
+// conv2_bias' v and the thread's target features tg.
+__device__ __forceinline__ void head_dots(const float (&v)[8], const float (&tg)[8], float& ss, float& dt) {
+  ss = 0.0f;
+  dt = 0.0f;
+#pragma unroll
+  for (int oo = 0; oo < 8; ++oo) { ss = fmaf(v[oo], v[oo], ss); dt = fmaf(v[oo], tg[oo], dt); }
+  ss = quad_sum(ss);
+  dt = quad_sum(dt);
+}
+
+// F.normalize: v / max(||v||, 1e-12); then <.,tgt> summed over channels, .mean(dim=-1) over the 64 positions.  Thread 0
+// stores the score to *out; red: the 8 floats of sm.red.  One __syncthreads.  The fp32 scorer and the gradient ascent
+// both score through here, so their scores agree bit for bit.
+__device__ __forceinline__ void mean_cosine(float ss, float dt, float* red, float* out) {
+  float cosv = ((threadIdx.x & 3) == 0) ? dt / fmaxf(sqrtf(ss), 1e-12f) : 0.0f;
+  cosv = warp_sum(cosv);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = cosv;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float tot = 0.0f;
+#pragma unroll
+    for (int w = 0; w < 8; ++w) tot += red[w];
+    *out = tot * (1.0f / 64.0f);
+  }
+}
+
 
 // One volume -> normalised features [32][64] (feat[o*64 + pos]); all 256 threads of the CTA.
 // Caller has staged the weights (stage_weights) and synchronised.

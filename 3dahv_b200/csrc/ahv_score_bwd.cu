@@ -25,9 +25,7 @@
 // it (counting sort over the <= 4096 contributions with integer shared-memory atomics and prefix sums), and every
 // thread walks the lists of its two input voxels - exactly the output voxels that touch them, whatever the matrix R
 // is - reading dX, which lies voxel-major with the channels innermost, as four LDS.128 per contribution.
-#include <cstddef>
-
-#include "ahv_head_fp32.cuh"
+#include "ahv_bwd_fp32.cuh"
 
 namespace ahv {
 
@@ -38,13 +36,8 @@ struct BwdSmem {
 };
 static_assert(sizeof(BwdSmem) <= 232448, "shared memory budget");
 
-// dX (gradient w.r.t. the rotated volume) overlays rotA / rotT once dW1 is done, voxel-major with the 16 channels
-// innermost: element (d, h, w, c) at d*kDxD + h*kDxH + w*kDxW + c floats - the adjoint reads a voxel's record as four
-// LDS.128.  The pitches are 4*odd mod 32: the fold's lanes (which run over h or over w) meet distinct bank groups.  The
-// adjoint's work list (<= 4096 entries of 8 bytes) follows it, into the dH1 buffer, which is dead by then as well.
-constexpr int kDxW = 20, kDxH = 164, kDxD = 1312, kDxFloats = 8 * kDxD;
-static_assert(offsetof(Fp32Smem, rotT) == offsetof(Fp32Smem, rotA) + sizeof(float) * kC * kRotC &&
-              offsetof(Fp32Smem, h1s) == offsetof(Fp32Smem, rotT) + sizeof(float) * kC * kRotC, "rotA, rotT, h1s are contiguous");
+// dX (ahv_bwd_fp32.cuh) overlays rotA / rotT once dW1 is done.  The adjoint's work list (<= 4096 entries of 8 bytes)
+// follows it, into the dH1 buffer, which is dead by then as well.
 static_assert((kDxFloats + 2 * kVox * 8) <= 2 * kC * kRotC + kP * kH1Row, "dX and the work list fit the dead buffers");
 static_assert(2 * kVox * sizeof(int) <= sizeof(float) * kP * kH1Row, "counters fit the dH2 buffer");
 static_assert((2 * kVox + 9 * kThreads / 32) * sizeof(float) <= sizeof(float) * kP * kH1Row,
@@ -159,31 +152,15 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
     }
     float v[8];
     conv2_bias(sm, b2r, v);
-    float ss = 0.0f, ft = 0.0f;
-#pragma unroll
-    for (int oo = 0; oo < 8; ++oo) { ss = fmaf(v[oo], v[oo], ss); ft = fmaf(v[oo], tg[oo], ft); }
-    ss = quad_sum(ss);
-    ft = quad_sum(ft);
-    {
-      // F = v / max(|v|, eps) (modules/modules.py:122).  d<F,T>/dv = (T - F <F,T>) / |v| above the clamp, T / eps below
-      const float nraw = sqrtf(ss), nr = fmaxf(nraw, 1e-12f), inv = 1.0f / nr;
-      const float fdot = ft * inv;  // <F, T>
-      const bool clamped = nraw < 1e-12f;
-#pragma unroll
-      for (int oo = 0; oo < 8; ++oo) {
-        const float F = v[oo] * inv;
-        const float d2 = g64 * inv * (clamped ? tg[oo] : tg[oo] - F * fdot);
-        aT[oo] = fmaf(g64, F, aT[oo]);
-        ab2[oo] += d2;
-        v[oo] = d2;
-      }
-      float* dst = bs.dh2 + pos * kH1Row + cg2 * 8;
-      *reinterpret_cast<float4*>(dst) = make_float4(v[0], v[1], v[2], v[3]);
-      *reinterpret_cast<float4*>(dst + 4) = make_float4(v[4], v[5], v[6], v[7]);
-    }
+    float ss, ft;
+    head_dots(v, tg, ss, ft);
+    head_dh2(v, tg, ss, ft, g64, bs.dh2, [&](int oo, float F, float d2) {
+      aT[oo] = fmaf(g64, F, aT[oo]);
+      ab2[oo] += d2;
+    });
     __syncthreads();
 
-    // ---------------- dW2 += dH2^T H1 ; dH1 = (dH2 W2) * [H1 > 0] ----------------
+    // ---------------- dW2 += dH2^T H1 ; dH1 = (dH2 W2) * [H1 > 0] (head_dh1) ----------------
     {
       const int o = t >> 3, i0 = (t & 7) * 4;
 #pragma unroll 8
@@ -194,32 +171,7 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
         aW2[2] = fmaf(d, h.z, aW2[2]); aW2[3] = fmaf(d, h.w, aW2[3]);
       }
     }
-    float dh1[8];
-    {
-      const int ig = cg2;  // input channels ig*8 .. +7 of position `pos`
-#pragma unroll
-      for (int j = 0; j < 8; ++j) dh1[j] = 0.0f;
-#pragma unroll 4
-      for (int o = 0; o < kO; ++o) {
-        const float d = bs.dh2[pos * kH1Row + o];
-        const float* wr = sm.w2s + ((o % 8) * 4 + o / 8) * kH1Row + ig * 8;  // W2[o][ig*8 ..]
-        const float4 w0 = *reinterpret_cast<const float4*>(wr), w1 = *reinterpret_cast<const float4*>(wr + 4);
-        dh1[0] = fmaf(d, w0.x, dh1[0]); dh1[1] = fmaf(d, w0.y, dh1[1]);
-        dh1[2] = fmaf(d, w0.z, dh1[2]); dh1[3] = fmaf(d, w0.w, dh1[3]);
-        dh1[4] = fmaf(d, w1.x, dh1[4]); dh1[5] = fmaf(d, w1.y, dh1[5]);
-        dh1[6] = fmaf(d, w1.z, dh1[6]); dh1[7] = fmaf(d, w1.w, dh1[7]);
-      }
-      const float* hp = sm.h1s + pos * kH1Row + ig * 8;  // ReLU mask (modules/modules.py:68)
-#pragma unroll
-      for (int j = 0; j < 8; ++j) dh1[j] = hp[j] > 0.0f ? dh1[j] : 0.0f;
-    }
-    __syncthreads();  // every dW2 read of h1s is done: overwrite it in place with dH1
-    {
-      float* hp = sm.h1s + pos * kH1Row + cg2 * 8;
-      *reinterpret_cast<float4*>(hp) = make_float4(dh1[0], dh1[1], dh1[2], dh1[3]);
-      *reinterpret_cast<float4*>(hp + 4) = make_float4(dh1[4], dh1[5], dh1[6], dh1[7]);
-    }
-    __syncthreads();
+    head_dh1(sm, bs.dh2, pos, cg2);
 
     // ---------------- dW1 += dH1^T A  (A = tri-plane views of the rotated volume) ----------------
     if (want_W1) {
@@ -250,62 +202,12 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
     __syncthreads();  // rotA / rotT are free: they become dX, voxel-major with the channels innermost
 
     // ---------------- dA = dH1 W1, folded view by view into dX ----------------
-    {
-      const int pl = t & 15, c = t >> 4;  // positions pl + 16 j, channel c, all (view, kk)
-      float* dX = sm.rotA + c;            // element (d, h, w, c) at d*kDxD + h*kDxH + w*kDxW + c
-#pragma unroll 1
-      for (int view = 0; view < 3; ++view) {
-        float acc[4][8];
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-#pragma unroll
-          for (int kk = 0; kk < 8; ++kk) acc[j][kk] = 0.0f;
-        const float* wv = sm.w1t + (view * 128 + c * 8) * kW1Pitch;
-#pragma unroll 2
-        for (int iq = 0; iq < 8; ++iq) {
-          float4 d[4];
-#pragma unroll
-          for (int j = 0; j < 4; ++j) d[j] = *reinterpret_cast<const float4*>(sm.h1s + (pl + 16 * j) * kH1Row + iq * 4);
-#pragma unroll
-          for (int kk = 0; kk < 8; ++kk) {
-            const float2 wa = *reinterpret_cast<const float2*>(wv + kk * kW1Pitch + iq * 4);
-            const float2 wb = *reinterpret_cast<const float2*>(wv + kk * kW1Pitch + iq * 4 + 2);
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-              acc[j][kk] = fmaf(d[j].x, wa.x, fmaf(d[j].y, wa.y, fmaf(d[j].z, wb.x, fmaf(d[j].w, wb.y, acc[j][kk]))));
-          }
-        }
-        // fold: every dX element gets exactly one contribution per view, so no races inside a view
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const int ps = pl + 16 * j, p = ps >> 3, q = ps & 7;
-#pragma unroll
-          for (int kk = 0; kk < 8; ++kk) {
-            if (view == 0) dX[p * kDxD + q * kDxH + kk * kDxW] = acc[j][kk];          // V'[c, d=p, h=q, w=kk]
-            else if (view == 1) dX[p * kDxD + kk * kDxH + q * kDxW] += acc[j][kk];    // V'[c, d=p, h=kk, w=q]
-            else dX[kk * kDxD + p * kDxH + q * kDxW] += acc[j][kk];                   // V'[c, d=kk, h=p, w=q]
-          }
-        }
-        __syncthreads();
-      }
-    }
+    fold_dA(sm, t);
 
-    // ---------------- dS/dR: the resampling differentiated in its grid (rot_grad_accum) ----------------
-    // dX (rotA, voxel-major, channels innermost), the halo'd source volume (sm.vol) and R (sm.Rcur, read from shared
-    // memory because the kernel runs at the register limit) are all in place.  Mapping of gather_hypothesis: 4 lanes
-    // per output voxel, 4 channels each.  The 9 partial sums meet in the dead dH2 buffer behind the adjoint's counters.
+    // ---------------- dS/dR: the resampling differentiated in its grid (rotation_grad) ----------------
+    // The 9 partial sums meet in the dead dH2 buffer behind the adjoint's counters.
     if (want_R) {
-      float G[9];
-#pragma unroll
-      for (int e = 0; e < 9; ++e) G[e] = 0.0f;
-      const int lane = t & 31, warp = t >> 5, j = lane & 3, w = lane >> 2;
-#pragma unroll 1
-      for (int pass = 0; pass < 8; ++pass) {
-        const int s = pass * 8 + warp, d = s >> 3, h = s & 7;
-        const float4 gx4 = *reinterpret_cast<const float4*>(sm.rotA + d * kDxD + h * kDxH + w * kDxW + 4 * j);
-        rot_grad_accum(sm.vol, sm.Rcur, sm.base[w], sm.base[h], sm.base[d], j, gx4, G);
-      }
-      const float sR = block_sum9(G, bs.dh2 + 2 * kVox, 4.0f);
+      const float sR = rotation_grad(sm, bs.dh2 + 2 * kVox, t);
       if (t < 9) {
         if (r_per_pair) g_R[(size_t)it * 9 + t] += sR;   // the item is this CTA's alone
         else atomicAdd(g_R + (size_t)n * 9 + t, sR);

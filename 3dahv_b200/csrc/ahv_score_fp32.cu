@@ -61,22 +61,9 @@ score_fp32_kernel(const T* __restrict__ vol_src, const float* __restrict__ tgt_f
     __syncthreads();
     float v[8];
     conv2_bias(sm, b2r, v);
-    float ss = 0.0f, dt = 0.0f;
-#pragma unroll
-    for (int oo = 0; oo < 8; ++oo) { ss = fmaf(v[oo], v[oo], ss); dt = fmaf(v[oo], tg[oo], dt); }
-    ss = quad_sum(ss);
-    dt = quad_sum(dt);
-    // F.normalize: v / max(||v||, 1e-12); then <.,tgt> summed over channels
-    float cosv = (cg2 == 0) ? dt / fmaxf(sqrtf(ss), 1e-12f) : 0.0f;
-    cosv = warp_sum(cosv);
-    if ((threadIdx.x & 31) == 0) sm.red[threadIdx.x >> 5] = cosv;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      float tot = 0.0f;
-#pragma unroll
-      for (int w = 0; w < 8; ++w) tot += sm.red[w];
-      scores[it] = tot * (1.0f / 64.0f);  // .mean(dim=-1) over 64 positions
-    }
+    float ss, dt;
+    head_dots(v, tg, ss, dt);
+    mean_cosine(ss, dt, sm.red, scores + it);
   }
 }
 

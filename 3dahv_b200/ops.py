@@ -423,6 +423,73 @@ def refine(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, m: int = 64, max_angle_
     return fv, fi, fR, cand, bv, bi, bR, workspace
 
 
+def _vol_src(vol_src):
+    if vol_src.dtype == torch.bfloat16:
+        return _dev(vol_src, "vol_src", torch.bfloat16), VOL_BF16
+    return _dev(vol_src, "vol_src"), VOL_F32
+
+
+def gradient_ascent(vol_src, tgt_feat, R_init, W1, W2, b2, steps: int = 20, step_deg: float = 1.0, out=None):
+    """ahv_gradient_ascent: backtracking Riemannian gradient ascent of the AHV_MATH_FP32 score on SO(3), every step of
+    every candidate in one launch.  vol_src [B,16,8,8,8] fp32|bf16, tgt_feat [B,32,64], R_init [B,K,3,3].  Returns
+    (R_out [B,K,3,3], score_out [B,K]); score_out is the fp32 scorer's score of R_out, never below that of R_init.
+    `out` = a previous result to write into (CUDA-graph replays)."""
+    vs, vdt = _vol_src(vol_src)
+    tf, R = _dev(tgt_feat, "tgt_feat"), _dev(R_init, "R_init")
+    B = vs.shape[0]
+    if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(tf.shape) != (B, 32, 64):
+        raise ValueError("vol_src [B,16,8,8,8] and tgt_feat [B,32,64] expected")
+    if R.dim() != 4 or R.shape[0] != B or tuple(R.shape[2:]) != (3, 3):
+        raise ValueError("R_init must be [B,K,3,3]")
+    W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+    K = R.shape[1]
+    if out is None:
+        out = (torch.empty(B, K, 3, 3, device=vs.device, dtype=torch.float32), torch.empty(B, K, device=vs.device, dtype=torch.float32))
+    R_out, s_out = out
+    base = base_coords(vs.device)
+    with torch.cuda.device(vs.device):
+        _lib.check(_lib.lib().ahv_gradient_ascent(vs.data_ptr(), vdt, tf.data_ptr(), R.data_ptr(), W1.data_ptr(), W2.data_ptr(),
+                                                  b2.data_ptr(), base.data_ptr(), int(steps), float(step_deg), R_out.data_ptr(),
+                                                  s_out.data_ptr(), B, K, _stream(vs)), "ahv_gradient_ascent")
+    return R_out, s_out
+
+
+def refine_gradient(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, steps: int = 20, step_deg: float = 1.0, math: int = MATH_TC,
+                    workspace: torch.Tensor | None = None, out=None):
+    """ahv_refine_gradient: top-k over the set, gradient ascent of the fp32 score from each winner, per-pair arg-max -
+    one C call, no torch ops, CUDA-graph capturable (pass `out` = the tuple a previous call returned to reuse its buffers).
+    Returns (first_val [B,k], first_idx [B,k], first_R [B,k,3,3], R_all [B,k,3,3], score_all [B,k], best_val [B],
+    best_idx [B], R_best [B,3,3], workspace)."""
+    vs, vdt = _vol_src(vol_src)
+    vt, R = _dev(vol_tgt, "vol_tgt"), _dev(R, "R")
+    B = vs.shape[0]
+    per_pair = R.dim() == 4
+    N = R.shape[1] if per_pair else R.shape[0]
+    if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
+        raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
+    if not 1 <= k <= min(32, N):
+        raise ValueError("1 <= k <= min(32, N) expected")
+    W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+    dev = vs.device
+    if out is None:
+        f = dict(device=dev, dtype=torch.float32)
+        out = (torch.empty(B, k, **f), torch.empty(B, k, device=dev, dtype=torch.int64), torch.empty(B, k, 3, 3, **f),
+               torch.empty(B, k, 3, 3, **f), torch.empty(B, k, **f), torch.empty(B, **f),
+               torch.empty(B, device=dev, dtype=torch.int64), torch.empty(B, 3, 3, **f))
+    fv, fi, fR, Ra, sa, bv, bi, bR = out[:8]
+    need = int(_lib.lib().ahv_refine_gradient_workspace_bytes(B, N, k))
+    if workspace is None or workspace.numel() * workspace.element_size() < need:
+        workspace = torch.empty(max(need, 16), device=dev, dtype=torch.uint8)
+    base = base_coords(dev)
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().ahv_refine_gradient(
+            vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
+            base.data_ptr(), k, int(steps), float(step_deg), fv.data_ptr(), fi.data_ptr(), fR.data_ptr(), Ra.data_ptr(),
+            sa.data_ptr(), bv.data_ptr(), bi.data_ptr(), bR.data_ptr(), B, N, math, workspace.data_ptr(),
+            workspace.numel() * workspace.element_size(), _stream(vs)), "ahv_refine_gradient")
+    return fv, fi, fR, Ra, sa, bv, bi, bR, workspace
+
+
 def _peer_array(peer):
     import ctypes
 

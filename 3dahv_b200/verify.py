@@ -120,7 +120,8 @@ class HypothesisVerifier:
         scores higher (theta *= 1.2 there, /= 2 elsewhere).  Candidates are scored with the fp32 kernel from start to
         end, so every returned score is >= its starting score.  A fixed number of steps, no host synchronisation:
         CUDA-graph capturable.  Returns (R_best [B,3,3], score [B], R_all [B,k,3,3], score_all [B,k]); the best is
-        the per-pair arg-max over k, ties to the lowest index."""
+        the per-pair arg-max over k, ties to the lowest index.
+        This is the torch-op restatement of the algorithm, kept as the reference for `ascend` (one kernel, faster)."""
         dev = vol_src.device
         W1, W2, b2 = self._weights_on(dev)
         R = (R_init[:, None] if R_init.dim() == 3 else R_init).float().contiguous()
@@ -152,6 +153,33 @@ class HypothesisVerifier:
         best = torch.argmax(s, dim=1)                                      # first maximal index
         rows = torch.arange(B, device=dev)
         return R[rows, best], s[rows, best], R, s
+
+    @torch.no_grad()
+    def ascend(self, vol_src, vol_tgt, R_init, steps: int = 20, step_deg: float = 1.0):
+        """`refine_gradient`'s ascent as one kernel (`ahv_gradient_ascent`): every step of every candidate runs on-chip,
+        one CTA per candidate at a time, and the score is differentiated again only where a trial was accepted.
+        R_init [B,3,3] or [B,k,3,3]; fp32 or bf16 source volumes.  Every returned score is the fp32 scorer's score of its
+        rotation and >= its starting score.  No host synchronisation: CUDA-graph capturable.  Returns (R_best [B,3,3],
+        score [B], R_all [B,k,3,3], score_all [B,k]); the best is the per-pair arg-max over k, ties to the lowest index."""
+        W1, W2, b2 = self._weights_on(vol_src.device)
+        R = (R_init[:, None] if R_init.dim() == 3 else R_init).float()
+        vs = vol_src if vol_src.dtype == torch.bfloat16 else vol_src.float()
+        R_all, s_all = ops.gradient_ascent(vs, self.target_features(vol_tgt), R, W1, W2, b2, steps=steps, step_deg=step_deg)
+        val, idx = ops.topk(s_all, 1)
+        return ops.gather_rotations(R_all, idx)[:, 0], val[:, 0], R_all, s_all
+
+    @torch.no_grad()
+    def refine_by_gradient(self, vol_src, vol_tgt, R, k: int = 32, steps: int = 20, step_deg: float = 1.0):
+        """Grid pass + gradient ascent in one C call (`ahv_refine_gradient`; BASELINE config 4's accurate path): score
+        the set with this verifier's math mode, keep the top-k, run `ascend` from each winner, return the best.
+        Returns (R_best [B,3,3], score [B], first pass as a VerifyResult, R_all [B,k,3,3], score_all [B,k])."""
+        W1, W2, b2 = self._weights_on(vol_src.device)
+        k = min(k, R.shape[1] if R.dim() == 4 else R.shape[0])
+        vs = vol_src if vol_src.dtype == torch.bfloat16 else vol_src.float()
+        fv, fi, fR, Ra, sa, bv, bi, bR, self._ws_refine_gradient = ops.refine_gradient(
+            vs, vol_tgt.float(), R, W1, W2, b2, k=k, steps=steps, step_deg=step_deg, math=self.math,
+            workspace=getattr(self, "_ws_refine_gradient", None))
+        return bR, bv, VerifyResult(None, fv, fi, fR), Ra, sa
 
 
 def _hat(u: torch.Tensor) -> torch.Tensor:
@@ -222,10 +250,15 @@ class GraphedRefiner:
     """CUDA-graph replay of the two-pass selection (`ahv_refine`: dense set -> top-k -> m local candidates each ->
     arg-max; BASELINE config 4) for fixed (B, N, k, m): the whole chain - target features, both scoring passes, top-k,
     candidate generation, selection - is one C call with no host step or torch op inside, so it captures as it stands.
+    method="gradient" captures `ahv_refine_gradient` instead (dense set -> top-k -> `steps` steps of gradient ascent
+    from each winner, starting at step_deg -> arg-max; m, max_angle_deg and seed are unused).
     Outputs are static tensors valid until the next replay."""
 
     def __init__(self, verifier: HypothesisVerifier, B: int, N: int, k: int = 32, m: int = 64, max_angle_deg: float = 5.0,
-                 seed: int = 0, device="cuda", vol_dtype=torch.float32):
+                 seed: int = 0, device="cuda", vol_dtype=torch.float32, method: str = "perturb", steps: int = 20,
+                 step_deg: float = 1.0):
+        if method not in ("perturb", "gradient"):
+            raise ValueError('method must be "perturb" or "gradient"')
         dev = torch.device(device)
         self.v = verifier.to(dev)
         self.vol_src = torch.zeros(B, 16, 8, 8, 8, device=dev, dtype=vol_dtype)
@@ -235,6 +268,9 @@ class GraphedRefiner:
         W1, W2, b2 = self.v._weights_on(dev)
 
         def run(out=None, ws=None):
+            if method == "gradient":
+                return ops.refine_gradient(self.vol_src, self.vol_tgt, self.R, W1, W2, b2, k=k, steps=steps, step_deg=step_deg,
+                                           math=self.v.math, workspace=ws, out=out)
             return ops.refine(self.vol_src, self.vol_tgt, self.R, W1, W2, b2, k=k, m=m, max_angle_deg=max_angle_deg, seed=seed,
                               math=self.v.math, workspace=ws, out=out)
 
@@ -242,19 +278,23 @@ class GraphedRefiner:
         stream.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(stream):
             res = run()
-            res = run(res[:7], res[7])             # warm-up on the buffers the graph will use
+            res = run(res[:-1], res[-1])           # warm-up on the buffers the graph will use
         torch.cuda.current_stream(dev).wait_stream(stream)
         torch.cuda.synchronize(dev)
-        self._bufs, self._ws = res[:7], res[7]
+        self._bufs, self._ws = res[:-1], res[-1]
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
             run(self._bufs, self._ws)
-        fv, fi, fR, self.candidates, self.best_val, self.best_idx, self.R_best = self._bufs
+        if method == "gradient":
+            fv, fi, fR, self.R_all, self.score_all, self.best_val, self.best_idx, self.R_best = self._bufs
+        else:
+            fv, fi, fR, self.candidates, self.best_val, self.best_idx, self.R_best = self._bufs
         self.first = VerifyResult(None, fv, fi, fR)
 
     @torch.no_grad()
     def __call__(self, vol_src=None, vol_tgt=None, R=None):
-        """Returns (R_best [B,3,3], score [B]); `.first` holds the first pass's top-k, `.candidates` the refinement set."""
+        """Returns (R_best [B,3,3], score [B]); `.first` holds the first pass's top-k, `.candidates` the refinement set
+        (method="perturb") or `.R_all` / `.score_all` the ascended top-k (method="gradient")."""
         if vol_src is not None:
             self.vol_src.copy_(vol_src, non_blocking=True)
         if vol_tgt is not None:

@@ -228,6 +228,31 @@ AHV_API int ahv_refine(const void* vol_src, int vol_dtype, const float* vol_tgt,
                        float* cand, float* best_val, int64_t* best_idx, float* R_best, int B, int64_t N,
                        int math_mode, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Gradient ascent of the AHV_MATH_FP32 score on SO(3) from given rotations (extension; the reference has none):
+ * R_init [B,K,3,3] per-pair candidates, tgt_feat [B,32,64] = ahv_forward_3d2d(vol_tgt).  `steps` backtracking steps
+ * starting at step_deg; R_out [B,K,3,3], score_out [B,K] = fp32 score of R_out, never below that of R_init.
+ * Each step forms a trial exp(theta [u]x) R along the Riemannian gradient direction u (then one Newton step back to
+ * SO(3)), keeps it only where it scores higher (theta *= 1.2 there, /= 2 elsewhere), and differentiates the score
+ * again only at an accepted trial.  vol_src fp32 or bf16 (AHV_VOL_*; bf16 is staged exactly: the same result as its
+ * fp32 copy).  The scores equal ahv_score(AHV_MATH_FP32) of R_out bit for bit, and the result is bit-deterministic.
+ * 0 <= steps <= 1000, step_deg finite and > 0; R_init / R_out 16-byte aligned.
+ * One launch, no host synchronisation, no allocation: CUDA-graph capturable. */
+AHV_API int ahv_gradient_ascent(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R_init,
+                                const float* W1, const float* W2, const float* b2, const float* base, int steps,
+                                float step_deg, float* R_out, float* score_out, int B, int K, void* stream);
+
+/* Grid -> top-k -> gradient ascent -> per-pair arg-max in one call (config 4's accurate path), like ahv_refine:
+ * ahv_verify(math_mode) keeps the top k (first_val/idx/R); ahv_gradient_ascent from first_R (R_all [B,k,3,3],
+ * score_all [B,k]); best_val [B], best_idx [B] (index into k, ties -> lowest), R_best [B,3,3] or NULL.
+ * k <= min(32, N); rotation buffers 16-byte aligned.  Workspace: ahv_refine_gradient_workspace_bytes.
+ * No host synchronisation, no allocation: CUDA-graph capturable. */
+AHV_API size_t ahv_refine_gradient_workspace_bytes(int B, int64_t N, int k);
+AHV_API int ahv_refine_gradient(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
+                                const float* W1, const float* W2, const float* b2, const float* base, int k, int steps,
+                                float step_deg, float* first_val, int64_t* first_idx, float* first_R, float* R_all,
+                                float* score_all, float* best_val, int64_t* best_idx, float* R_best, int B, int64_t N,
+                                int math_mode, void* workspace, size_t workspace_bytes, void* stream);
+
 /* torch.max / top-k over an existing score matrix (modules/model.py:195). */
 AHV_API int ahv_topk(const float* scores, int B, int64_t N, int k, int64_t idx_offset, float* topk_val,
              int64_t* topk_idx, void* workspace, size_t workspace_bytes, void* stream);
