@@ -37,6 +37,36 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// Largest L1 norm of a row of W ([32 rows][kCols], fp32), by `kWarps` warps: warp w sums rows w, w + kWarps, ...  Each
+// row's sum has one fixed order (lane partial sums, then the butterfly) whatever kWarps is, so every CTA of the tensor-core
+// scoring kernel and of the tcgen05 backward derives the same value.
+template <int kCols, int kWarps>
+__device__ __forceinline__ float row_l1max(const float* __restrict__ W, int warp, int lane) {
+  constexpr int kRowsPerWarp = (kO + kWarps - 1) / kWarps;
+  float m = 0.0f;
+#pragma unroll
+  for (int i = 0; i < kRowsPerWarp; ++i) {
+    const int r = warp + i * kWarps;
+    if (r < kO) {
+      float l1 = 0.0f;
+#pragma unroll
+      for (int j = 0; j < kCols / 32; ++j) l1 += fabsf(__ldg(W + r * kCols + lane + 32 * j));
+      m = fmaxf(m, warp_sum(l1));
+    }
+  }
+  return m;  // this warp's largest row norm (identical in all lanes)
+}
+
+// Power-of-two normalisation of a weight matrix: e = floor(log2 of its largest row L1 norm) - `target`, so that W * 2^-e
+// has that norm in [2^target, 2^(target+1)) whatever the weights' magnitude.  0 when the weights are all zero or not
+// finite.
+__device__ __forceinline__ int weight_exponent(float l1max, int target) {
+  return (l1max > 0.0f && isfinite(l1max)) ? max(-60, min(60, ilogbf(l1max) - target)) : 0;
+}
+// W1's normalised row norms land in [4, 8), which keeps the tensor-core scorer's pair-scaled volume in (2^11, 2^13]
+// (stage_pair_volume); W2's land in [1, 2) (conv2 accumulates in fp32; only its fp16 operand needs the range).
+constexpr int kW1NormTarget = 2, kW2NormTarget = 0;
+
 // Sample position of output voxel (x,y,z base coordinates) under rotation R
 // (F.affine_grid, utils.py:126), un-normalised as grid_sample does with
 // align_corners=False: i = ((g+1)*8-1)/2.  ((g+1)*8 is exact, so one FFMA

@@ -28,9 +28,11 @@
 //                                                      its (d,h) one
 //   dH1, dH2^T, H1^T  [ch][pos] : SBO 1040, LBO 128    B of dW1, A and B of dW2 (pitch 1040: the eight 2-byte stores of a
 //                                                      thread's channel block hit distinct banks across the warp)
-// Scales (powers of two, undone in fp32 when the accumulators are read): H1 and A^T carry the pair's scale of the
-// forward (pair_inv_scale); dH2 a per-item scale from the bound 2 |g/64| / min_p |H2_p|; dH1 a per-item scale from
-// max |dH1| (2^13 <= max < 2^14); dX (fp16) a launch-wide one from W1's largest column L1 norm.
+// Scales (powers of two, undone in fp32 when the accumulators are read): W1 and W2 are packed as W * 2^-e (largest row
+// L1 norm in [4, 8) / [1, 2)), as the forward packs them (same sums, same e); H1 carries the forward's pair scale s and
+// W1's normaliser (pair_inv_scale = 2^e1 / s), A^T the pair scale s alone; dH2 a per-item scale from the bound
+// 2 |g/64| / min_p |H2_p|; dH1 a per-item scale from max |dH1| (2^13 <= max < 2^14); dX (fp16) a launch-wide one, kappa,
+// from the normalised W1's largest column L1 norm (inv_kappa also undoes 2^-e1).
 // The M=64 accumulators come in pairs side by side in the lanes (lanes 0-15 / 16-31 of every 32-lane quadrant hold two
 // column blocks of the same 16 rows), so all 32 lanes of a warp read; dW1^T and dW2 are read every item into per-thread
 // fp32 accumulators (48 + 8), which keeps the accumulation across items in fp32 and lets the scales differ per item.
@@ -76,8 +78,9 @@ constexpr int kColH2 = 288, kColDh1 = 304, kColW2 = 320;   // conv2, dH1, dW2 ac
 // channels innermost, in fp16: the adjoint's random reads of it are what bounds the kernel, and a record of 32 bytes
 // costs half the shared-memory wavefronts of an fp32 one.  Element (d, h, w, c) at word d*kDxD + h*kDxH + w*kDxW + c/2
 // (pitches in 4-byte words, multiples of 4 so that a record is two aligned LDS.128).  The values are the raw
-// accumulators (dH1's per-item scale S) times kappa, a power of two fixed per launch from W1 so that the sum of the
-// three views cannot overflow fp16: |dA| S < 2^14 * max_k sum_o |W1[o][k]|, kappa <= 2 / (3 * that maximum).
+// accumulators (dH1's per-item scale S, W1's normaliser 2^-e1) times kappa, a power of two fixed per launch from the
+// packed W1 so that the sum of the three views cannot overflow fp16: |acc| < 2^14 * max_k sum_o |fp16(W1[o][k] 2^-e1)|,
+// kappa <= 2 / (3 * that maximum).
 constexpr int kDxW = 12, kDxH = 100, kDxD = 804;
 static_assert(8 * kDxD * 4 <= kAtBytes, "dX fits over the A^T operand");
 
@@ -243,25 +246,38 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
   asm volatile("mov.u32 %0, %1;" : "=r"(sbase) : "r"(smem_u32(smem_raw)));
   const uint32_t bar_s = sbase + (uint32_t)offsetof(BwdTcSmem, bar);
 
-  // ---- set-up: W2 (fp32), W1^T operand (fp16, permuted rows), base coordinates, barrier, TMEM ----
-  for (int i = t; i < kO * kO; i += kThreads) {
-    const int o = i / kO, c = i % kO;
-    const __half w = __float2half_rn(__ldg(W2 + i));
+  // ---- set-up: weight normalisers, W2 operands, W1^T operand (fp16, permuted rows), base coordinates, barrier, TMEM ----
+  sm.part[warp] = make_float2(row_l1max<kK, kThreads / 32>(W1, warp, lane), row_l1max<kO, kThreads / 32>(W2, warp, lane));
+  __syncthreads();
+  float n1, w1s, w2s;   // 2^-e1, 2^e1, 2^e2
+  {
+    float m1 = sm.part[0].x, m2 = sm.part[0].y;
+#pragma unroll
+    for (int w = 1; w < kThreads / 32; ++w) { m1 = fmaxf(m1, sm.part[w].x); m2 = fmaxf(m2, sm.part[w].y); }
+    const int e1 = weight_exponent(m1, kW1NormTarget), e2 = weight_exponent(m2, kW2NormTarget);
+    n1 = scalbnf(1.0f, -e1);
+    w1s = scalbnf(1.0f, e1);
+    w2s = scalbnf(1.0f, e2);
+    const float n2 = scalbnf(1.0f, -e2);
+    for (int i = t; i < kO * kO; i += kThreads) {
+      const int o = i / kO, c = i % kO;
+      const __half w = __float2half_rn(__ldg(W2 + i) * n2);
     *reinterpret_cast<__half*>(sm.w2b + (o >> 3) * 512 + (c >> 3) * 128 + (o & 7) * 16 + (c & 7) * 2) = w;   // rows o, K = i
-    *reinterpret_cast<__half*>(sm.w2tb + (c >> 3) * 512 + (o >> 3) * 128 + (c & 7) * 16 + (o & 7) * 2) = w;  // rows i, K = o
+      *reinterpret_cast<__half*>(sm.w2tb + (c >> 3) * 512 + (o >> 3) * 128 + (c & 7) * 16 + (o & 7) * 2) = w;  // rows i, K = o
+    }
   }
   for (int i = t; i < kO * kK; i += kThreads) {
     const int o = i / kK, k = i - o * kK;  // coalesced read of W1[o][k]
     const int view = k >> 7, c = (k >> 3) & 15, kk = k & 7;
     const int grp = (c >> 2) * 12 + view * 4 + (c & 3);  // n' / 8
-    *reinterpret_cast<__half*>(sm.w1t + grp * 512 + (o >> 3) * 128 + kk * 16 + (o & 7) * 2) = __float2half_rn(__ldg(W1 + i));
+    *reinterpret_cast<__half*>(sm.w1t + grp * 512 + (o >> 3) * 128 + kk * 16 + (o & 7) * 2) = __float2half_rn(__ldg(W1 + i) * n1);
   }
   if (t < 8) sm.base[t] = base ? base[t] : 0.0f;
-  {  // largest L1 norm of a W1 column (fp16-rounded, as the MMA sees it): bounds |dA| / max|dH1| for the fp16 dX
+  {  // largest L1 norm of a packed W1 column (normalised, fp16-rounded, as the MMA sees it): bounds |dA acc| / max|dH1 S|
     float cmax = 0.0f;
     for (int k = t; k < kK; k += kThreads) {
       float c1 = 0.0f;
-      for (int o = 0; o < kO; ++o) c1 += fabsf(__half2float(__float2half_rn(__ldg(W1 + o * kK + k))));
+      for (int o = 0; o < kO; ++o) c1 += fabsf(__half2float(__float2half_rn(__ldg(W1 + o * kK + k) * n1)));
       cmax = fmaxf(cmax, c1);
     }
 #pragma unroll
@@ -283,7 +299,7 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = sm.tmem_slot;
-  float kappa = 1.0f, inv_kappa = 1.0f;
+  float kappa = 1.0f, inv_kappa = w1s;   // dX = acc * kappa; dA = dX * inv_kappa / S (inv_kappa undoes W1's normaliser too)
   {
     float c = sm.red[0];
 #pragma unroll
@@ -292,7 +308,7 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
       const float x = 2.0f / (3.0f * c);
       const int e = min(max(((__float_as_int(x) >> 23) & 0xff) - 127, -60), 60);   // floor(log2 x)
       kappa = __int_as_float((127 + e) << 23);
-      inv_kappa = __int_as_float((127 - e) << 23);
+      inv_kappa = __int_as_float((127 - e) << 23) * w1s;
     }
   }
   const uint32_t at_s = sbase + (uint32_t)offsetof(BwdTcSmem, at), w1t_s = sbase + (uint32_t)offsetof(BwdTcSmem, w1t);
@@ -383,7 +399,7 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
   };
 
   int cur_b = -1;
-  float pinv = 1.0f;
+  float pinv = 1.0f, pvol = 1.0f;   // H1 = h1 * pinv (2^e1 / s); 1/s, the volume's scale in A^T
   uint32_t phase = 0;
   float r_next = 0.0f;
   if (t < 9) r_next = __ldg(R + (r_per_pair ? (size_t)lo : (size_t)(lo % N)) * 9 + t);
@@ -399,6 +415,7 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
 #pragma unroll
       for (int oo = 0; oo < 8; ++oo) tg[oo] = tgt_feat[((size_t)b * kO + cg2 * 8 + oo) * kP + pos];
       pinv = __ldg(pair_inv + b);
+      pvol = pinv * n1;
       cur_b = b;
     }
     cnt[t] = 0;   // the work list's counters (the previous item's adjoint is behind a barrier)
@@ -445,7 +462,7 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
       }
       __syncwarp();
     }
-    pack_views(sm, 1.0f / pinv);
+    pack_views(sm, 1.0f / pvol);
     AHV_PH(2);
     mbar_wait(bar_s + 8, phase);
     tc_fence_after();
@@ -455,7 +472,9 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
       tmem_ld8(tq + kColH2 + hf * 8, r8);
       tmem_ld_wait();
 #pragma unroll
-      for (int oo = 0; oo < 8; ++oo) v[oo] = fmaf(__uint_as_float(r8[oo]), pinv, b2r[oo]);  // undo the pair scale, add bias
+      const float sc = pinv * w2s;   // undo the pair scale and both weight normalisers
+#pragma unroll
+      for (int oo = 0; oo < 8; ++oo) v[oo] = fmaf(__uint_as_float(r8[oo]), sc, b2r[oo]);  // + bias
     }
     float ss = 0.0f, ft = 0.0f;
 #pragma unroll
@@ -543,9 +562,10 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
       const uint4 hm = *reinterpret_cast<const uint4*>(sm.h1a + (pos >> 3) * 512 + cg2 * 128 + (pos & 7) * 16);
       const __half* hp = reinterpret_cast<const __half*>(&hm);  // ReLU mask (modules/modules.py:68)
       float mx = 0.0f;
+      const float dsc = inv_s2 * w2s;   // undo the dH2 scale and W2's normaliser
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
-        dh1[j] = __half2float(hp[j]) > 0.0f ? __uint_as_float(r8[j]) * inv_s2 : 0.0f;
+        dh1[j] = __half2float(hp[j]) > 0.0f ? __uint_as_float(r8[j]) * dsc : 0.0f;
         mx = fmaxf(mx, fabsf(dh1[j]));
       }
 #pragma unroll
@@ -616,7 +636,7 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
     phase ^= 1;
     tc_fence_after();
     {
-      const float sc = invS * pinv;  // undo the item's dH1 scale and the pair's volume scale
+      const float sc = invS * pvol;  // undo the item's dH1 scale and the pair's volume scale
       uint32_t r[16];
 #pragma unroll
       for (int view = 0; view < 3; ++view) {
@@ -657,7 +677,7 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
         for (int kk = 0; kk < 8; ++kk) add4_record(dst + kk * kDxD, kappa, r[kk], r[8 + kk], r[16 + kk], r[24 + kk]);
       }
     }
-    const float unscale = invS * inv_kappa;   // dX holds dA * S * kappa
+    const float unscale = invS * inv_kappa;   // dX holds dA * S * 2^-e1 * kappa
     __syncthreads();
     AHV_PH(8);
 

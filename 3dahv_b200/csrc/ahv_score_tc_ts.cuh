@@ -74,14 +74,15 @@ score_tc_ts_kernel(const __grid_constant__ CUtensorMap vol_map, const float* __r
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + M::off_misc);
   float* partial = reinterpret_cast<float*>(smem + M::off_misc + 16);  // [2 tilebuf][2 slot][4 warps]
   float* sbase = reinterpret_cast<float*>(smem + M::off_misc + 96);    // 8 base coordinates
-  uint32_t* l1max_bits = reinterpret_cast<uint32_t*>(smem + M::off_misc + 128);  // max L1 norm of a W1 row (float bits)
+  uint32_t* l1max_bits = reinterpret_cast<uint32_t*>(smem + M::off_misc + 128);  // max L1 row norms (float bits): W1, W2 for
+                                                                                 // pack_weights, W1 for the gather's pair scale
   float* red = reinterpret_cast<float*>(smem + M::off_misc + 144);        // 8 per-warp maxima (volume staging)
   float* inv_ring = reinterpret_cast<float*>(smem + M::off_misc + 176);   // 1/scale of pair b at [b & 7] (gather -> epilogue)
 
   for (int i = threadIdx.x; i < kVolSmemBytes / 16; i += kThreadsTC)
     reinterpret_cast<uint4*>(vol)[i] = make_uint4(0, 0, 0, 0);  // halo stays zero for the whole kernel
   if (threadIdx.x < 8) sbase[threadIdx.x] = base[threadIdx.x];
-  if (threadIdx.x == 8) *l1max_bits = 0u;
+  if (threadIdx.x >= 8 && threadIdx.x < 11) l1max_bits[threadIdx.x - 8] = 0u;
   // ---- source volumes by TMA (cp.async.bulk.tensor, 3-D map over [B*16 ch][8 d][64 hw]; one box = one pair's
   // volume, 32 KB fp32 / 16 KB bf16).  The box of the pair that starts at tile t lands in A-operand stage buffer
   // t % kStages - idle at that moment: the tensor core finished reading it with tile t-3 and the gather fills it only
@@ -128,8 +129,9 @@ score_tc_ts_kernel(const __grid_constant__ CUtensorMap vol_map, const float* __r
   tc_fence_after();
   const uint32_t tmem = *tmem_slot;
   if (threadIdx.x == 0) AHV_TL(1);
+  WeightScale wscale;
   if (warp >= kGatherWarps) {  // MMA + epilogue warps: weights -> fp16 operand layouts, then release the MMA warp
-    pack_weights(smem + M::off_w1, W1, W2, threadIdx.x - kGatherWarps * 32);
+    wscale = pack_weights(smem + M::off_w1, W1, W2, l1max_bits, threadIdx.x - kGatherWarps * 32);
     fence_proxy_async();  // written through the generic proxy, UMMA reads through the async proxy
     named_bar_sync(3, kPackThreads);
     if (threadIdx.x == 256) AHV_TL(5);
@@ -193,12 +195,9 @@ score_tc_ts_kernel(const __grid_constant__ CUtensorMap vol_map, const float* __r
       // first rotations
       cur_b = fb;
       const float inv = stage_pair_volume<T, K16>(smem + M::off_vol, reinterpret_cast<const T*>(smem + M::off_a),
-                                                  bar0 + kVolFull * 8, 0, l1max_bits, W1, true, red, gtid);
+                                                  bar0 + kVolFull * 8, 0, l1max_bits + 2, W1, true, red, gtid);
       ++vol_uses;
-      if (gtid == 0) {
-        inv_ring[fb & 7] = inv;
-        if constexpr (kSave) fin.pair_inv_out[fb] = inv;   // the same value from every CTA that stages this pair
-      }
+      if (gtid == 0) inv_ring[fb & 7] = inv;
       named_bar_sync(1, kGatherWarps * 32);
       if (threadIdx.x == 0) AHV_TL(3);
 #pragma unroll
@@ -298,13 +297,10 @@ score_tc_ts_kernel(const __grid_constant__ CUtensorMap vol_map, const float* __r
         named_bar_sync(1, kGatherWarps * 32);
         // requested two tiles ago, into the stage buffer THIS tile is about to fill
         const float inv = stage_pair_volume<T, K16>(smem + M::off_vol, reinterpret_cast<const T*>(smem + M::off_a + (g % kStages) * M::tile_bytes),
-                                                    bar0 + (kVolFull + (vol_uses & 1)) * 8, (vol_uses >> 1) & 1, l1max_bits, W1, false,
+                                                    bar0 + (kVolFull + (vol_uses & 1)) * 8, (vol_uses >> 1) & 1, l1max_bits + 2, W1, false,
                                                     red, gtid);
         ++vol_uses;
-        if (gtid == 0) {
-          inv_ring[it.b & 7] = inv;
-          if constexpr (kSave) fin.pair_inv_out[it.b] = inv;
-        }
+        if (gtid == 0) inv_ring[it.b & 7] = inv;
         named_bar_sync(1, kGatherWarps * 32);
         cur_b = it.b;
       }
@@ -468,7 +464,7 @@ score_tc_ts_kernel(const __grid_constant__ CUtensorMap vol_map, const float* __r
     __syncwarp();
   } else {
     // =========================== EPILOGUE ===========================
-    epilogue_role<kSave>(work, warp - kEpiWarp0, lane, tmem, bar0, M::tmem_a2, partial, tgt_feat, b2, inv_ring,
+    epilogue_role<kSave>(work, warp - kEpiWarp0, lane, tmem, bar0, M::tmem_a2, partial, tgt_feat, b2, inv_ring, wscale,
                         scores, best_keys, N, B, R, r_per_pair, fin);
   }
 

@@ -52,9 +52,10 @@ struct Finalize {
   float* R_best = nullptr;
   int64_t idx_offset = 0;
   unsigned* counter = nullptr;  // zero at kernel start (cleared with the keys), reset by the last CTA
-  // training forward (kSave instantiation only): conv1's ReLU'd output of every item, fp16 in the pair's scaled units
-  // [B*N][64 positions][32 channels], and 1/scale per pair - the fused backward reads them instead of recomputing
-  // conv1 (4 KB per item; the reference's autograd saves ~420 KB per hypothesis)
+  // training forward (kSave instantiation only): conv1's ReLU'd output of every item, fp16 in the units the kernel
+  // computed it in (pair scale s, normalised W1) [B*N][64 positions][32 channels], and per pair the factor that turns
+  // it back into conv1's output, 2^e1 / s - the fused backward reads them instead of recomputing conv1 (4 KB per
+  // item; the reference's autograd saves ~420 KB per hypothesis)
   __half* h1_out = nullptr;
   float* pair_inv_out = nullptr;
   // hypothesis set sharded over `peers.world` GPUs (SURVEY.md §8e): the winners are exchanged through peer
@@ -176,14 +177,32 @@ struct TileIter {
   }
 };
 
-// ---- one-time per CTA: W1/W2 (fp32, global) -> fp16 UMMA B-operand layouts in shared memory ------------
+// What undoes the normalisation: 2^e1 (conv1's output = its normalised form * w1) and 2^(e1+e2) (conv2's)
+struct WeightScale {
+  float w1 = 1.0f, w12 = 1.0f;
+};
+
+// ---- one-time per CTA: W1/W2 (fp32, global) -> normalised fp16 UMMA B-operand layouts in shared memory ------------
 // conv1: 24 slices j = (view, kk), each [chalf][ngroup][n%8][c%8]; conv2: [kc][ngroup][8][8] behind them.
-// Every CTA does this itself (52 KB of L2 reads) so that the scoring kernel depends on no preparation
-// kernel.  It runs on the 5 non-gather warps (MMA + epilogue, tid = 0..159) while the gather warps already
-// stage the first volume and resample the first tile; the MMA warp is released by named barrier 3.
+// Every CTA does this itself (52 KB of L2 reads, twice) so that the scoring kernel depends on no preparation kernel.
+// It runs on the 5 non-gather warps (MMA + epilogue, tid = 0..159) while the gather warps already stage the first
+// volume and resample the first tile; the MMA warp is released by named barrier 3.  l1max_bits[2] (zero on entry)
+// collects the row-norm maxima of W1 and W2 (a non-negative float's bit pattern orders like the float).
 constexpr int kPackThreads = kThreadsTC - kGatherWarps * 32;  // 160
-__device__ __forceinline__ void pack_weights(unsigned char* wsm, const float* __restrict__ W1,
-                                             const float* __restrict__ W2, int tid) {
+__device__ __forceinline__ WeightScale pack_weights(unsigned char* wsm, const float* __restrict__ W1,
+                                                    const float* __restrict__ W2, uint32_t* l1max_bits, int tid) {
+  {
+    const int warp = tid >> 5, lane = tid & 31;
+    const float m1 = row_l1max<kK, kPackThreads / 32>(W1, warp, lane), m2 = row_l1max<kO, kPackThreads / 32>(W2, warp, lane);
+    if (lane == 0) {
+      atomicMax(l1max_bits, __float_as_uint(m1));
+      atomicMax(l1max_bits + 1, __float_as_uint(m2));
+    }
+    named_bar_sync(3, kPackThreads);
+  }
+  const int e1 = weight_exponent(__uint_as_float(l1max_bits[0]), kW1NormTarget);
+  const int e2 = weight_exponent(__uint_as_float(l1max_bits[1]), kW2NormTarget);
+  const float n1 = scalbnf(1.0f, -e1), n2 = scalbnf(1.0f, -e2);
   __half* w1h = reinterpret_cast<__half*>(wsm);
   constexpr int kV4 = kO * kK / 4;  // float4 = 4 consecutive kk of one (row, view, channel)
 #pragma unroll 10
@@ -192,34 +211,17 @@ __device__ __forceinline__ void pack_weights(unsigned char* wsm, const float* __
     const int n = i / (kK / 4), k = (i - n * (kK / 4)) * 4;
     const int view = k >> 7, c = (k >> 3) & 15, kk = k & 7;
     __half* dst = w1h + (view * 8 + kk) * 512 + (c >> 3) * 256 + (n >> 3) * 64 + (n & 7) * 8 + (c & 7);
-    dst[0] = __float2half_rn(w4.x); dst[512] = __float2half_rn(w4.y);
-    dst[1024] = __float2half_rn(w4.z); dst[1536] = __float2half_rn(w4.w);
+    dst[0] = __float2half_rn(w4.x * n1); dst[512] = __float2half_rn(w4.y * n1);
+    dst[1024] = __float2half_rn(w4.z * n1); dst[1536] = __float2half_rn(w4.w * n1);
   }
   for (int i = tid; i < kO * kO; i += kPackThreads) {
     const int n = i / kO, k = i % kO;
-    w1h[kW1Bytes / 2 + (k >> 3) * 256 + (n >> 3) * 64 + (n & 7) * 8 + (k & 7)] = __float2half_rn(__ldg(W2 + i));
+    w1h[kW1Bytes / 2 + (k >> 3) * 256 + (n >> 3) * 64 + (n & 7) * 8 + (k & 7)] = __float2half_rn(__ldg(W2 + i) * n2);
   }
-}
-
-// Largest L1 norm of a W1 row (bounds |conv1 output| / max|V| for the pair scale), by the 8 gather warps:
-// warp w sums rows 4w..4w+3 (48 coalesced loads per lane in flight, fixed summation order -> the same value
-// in every CTA); the caller folds the per-warp maxima into *l1max_bits (a non-negative float's bit pattern orders
-// like the float).
-__device__ __forceinline__ float w1_l1max_partial(const float* __restrict__ W1, int warp, int lane) {
-  float wv[4][12];
-#pragma unroll
-  for (int r = 0; r < 4; ++r)
-#pragma unroll
-    for (int j = 0; j < 12; ++j) wv[r][j] = __ldg(W1 + (4 * warp + r) * kK + lane + 32 * j);
-  float m = 0.0f;
-#pragma unroll
-  for (int r = 0; r < 4; ++r) {
-    float l1 = 0.0f;
-#pragma unroll
-    for (int j = 0; j < 12; ++j) l1 += fabsf(wv[r][j]);
-    m = fmaxf(m, warp_sum(l1));
-  }
-  return m;  // this warp's largest row norm (identical in all lanes)
+  WeightScale ws;
+  ws.w1 = scalbnf(1.0f, e1);
+  ws.w12 = scalbnf(1.0f, e1 + e2);
+  return ws;
 }
 
 // ---- per pair: stage the source volume, pre-scaled by the pair's power-of-two scale -------------------
@@ -227,8 +229,13 @@ __device__ __forceinline__ float w1_l1max_partial(const float* __restrict__ W1, 
 // ([16 ch][512 voxels], fp32 or bf16), brought into shared memory by TMA (a 3-D tensor-map copy issued one tile
 // before the pair switch, landing in the A-operand stage the next tile will use; completion on mbarrier
 // `bar_vol`, phase `parity`).  The volume is read once into registers, its
-// max |V| reduced over the 8 warps, the scale s = 2^e chosen so that max|V|*s <= 2^12 and
-// max|V|*s*L1max <= 2^14 (fp16 max 65504; exact, undone after conv2), then the scaled values are written in
+// max |V| reduced over the 8 warps, the scale s = 2^e chosen so that max|V|*s lies in (b/2, b] (exact, undone after
+// conv2), b = 2^15 / L1n with L1n the largest row L1 norm of the normalised W1 (in [4, 8), see pack_weights): conv1's
+// output |H1| <= max|V|*s*L1n then lies in (2^14, 2^15] for the pair's largest voxel - as far above fp16's subnormals as
+// its maximum (65504) allows - and b in (2^12, 2^13] depends on W1's mantissa only, not on its magnitude.  (It used to
+// be min(2^12, 2^14 / L1max) of the raw W1, which cost the volume a bit of headroom per factor of 2 in W1.)  W1's row
+// norms are summed here too (the same sums as pack_weights', which runs concurrently), folded into *l1max_bits (a
+// non-negative float's bit pattern orders like the float).  Then the scaled values are written in
 // the gather's layout: fp32 lines [halo voxel][16 ch], or for 16-bit "x-pair lines" (every voxel is tap 0 of
 // pair xh and tap 1 of pair xh-1).  Returns 1/s.
 template <typename T>
@@ -246,8 +253,8 @@ __device__ AHV_STAGE_INLINE float stage_pair_volume(unsigned char* vsm, const T*
                                                    uint32_t* l1max_bits, const float* __restrict__ W1, bool first,
                                                    float* red, int gtid) {
   float wnorm = 0.0f;
-  if (first) wnorm = w1_l1max_partial(W1, gtid >> 5, gtid & 31);  // W1 row norms: in flight while the TMA lands
-  mbar_wait(bar_vol, parity);                                      // the pair's volume is in shared memory
+  if (first) wnorm = row_l1max<kK, kGatherWarps>(W1, gtid >> 5, gtid & 31);  // W1 row norms: in flight while the TMA lands
+  mbar_wait(bar_vol, parity);                                                  // the pair's volume is in shared memory
   float val[32];
 #pragma unroll
   for (int i = 0; i < 32; ++i) {
@@ -272,7 +279,8 @@ __device__ AHV_STAGE_INLINE float stage_pair_volume(unsigned char* vsm, const T*
   for (int w = 1; w < kGatherWarps; ++w) m = fmaxf(m, red[w]);
   float sc = 1.0f;
   if (m > 0.0f && isfinite(m)) {
-    const float bound = fminf(4096.0f, 16384.0f / fmaxf(l1max, 1e-20f));
+    const float l1n = scalbnf(l1max, -weight_exponent(l1max, kW1NormTarget));
+    const float bound = fminf(8192.0f, 32768.0f / fmaxf(l1n, 1e-20f));
     int e = ilogbf(bound / m);  // floor(log2)
     e = max(-100, min(100, e));
     sc = scalbnf(1.0f, e);
@@ -312,14 +320,14 @@ __device__ AHV_STAGE_INLINE float stage_pair_volume(unsigned char* vsm, const T*
 // 4 warps, warp s = TMEM sub-partition s.  Per hypothesis pair (tile):
 //   phase A: tcgen05.ld D1 -> ReLU (modules/modules.py:68) -> fp16 -> conv2's A operand, straight into TMEM
 //            (tcgen05.st; conv2 runs in the TS form);
-//   phase B (one tile later, after conv2): tcgen05.ld D2 -> undo the pair scale, + bias -> L2 norm with
+//   phase B (one tile later, after conv2): tcgen05.ld D2 -> undo the pair and weight scales, + bias -> L2 norm with
 //            F.normalize's eps (:122) -> dot with the target features (registers) -> mean over the 64
 //            positions (modules/model.py:193) -> score, and the running arg-max key (:195).
 template <bool kSave = false>
 __device__ __forceinline__ void epilogue_role(const Work& work, int s, int lane, uint32_t tmem, uint32_t bar0,
                                               uint32_t tmem_a2, float* partial,
                                               const float* __restrict__ tgt_feat, const float* __restrict__ b2,
-                                              const float* inv_ring, float* __restrict__ scores,
+                                              const float* inv_ring, WeightScale ws, float* __restrict__ scores,
                                               u64* __restrict__ best_keys, int64_t N, int B,
                                               const float* __restrict__ R, int r_per_pair, const Finalize& fin) {
   const int slot = lane >> 4;            // which hypothesis of the tile
@@ -353,7 +361,7 @@ __device__ __forceinline__ void epilogue_role(const Work& work, int s, int lane,
     float ss = 0.0f, dt = 0.0f;
 #pragma unroll
     for (int o = 0; o < kO; ++o) {
-      const float v = fmaf(__uint_as_float(r[o]), pinv, b2r[o]);  // undo the pair scale, add bias
+      const float v = fmaf(__uint_as_float(r[o]), pinv, b2r[o]);  // undo the pair and weight scales, add bias
       ss = fmaf(v, v, ss);
       dt = fmaf(v, tg[o], dt);
     }
@@ -414,7 +422,11 @@ __device__ __forceinline__ void epilogue_role(const Work& work, int s, int lane,
     if (g > 0) phase_b(g - 1, prev_b, prev_n0, prev_cnt, prev_inv);
     if (it.b != cur_b) {  // target features / scale of the tile just handed to conv2
       cur_b = it.b;
-      inv_s = inv_ring[cur_b & 7];  // written by the gather role when it staged this pair
+      const float inv_pair = inv_ring[cur_b & 7];  // 1/s, written by the gather role when it staged this pair
+      inv_s = inv_pair * ws.w12;                   // conv2's output = D2 * 2^(e1+e2) / s (powers of two: exact)
+      if constexpr (kSave) {                       // the same value from every CTA that scores this pair
+        if (s == 0 && lane == 0) fin.pair_inv_out[cur_b] = inv_pair * ws.w1;
+      }
 #pragma unroll
       for (int o = 0; o < kO; ++o) tg[o] = __ldg(tgt_feat + ((size_t)cur_b * kO + o) * kP + pos);
     }

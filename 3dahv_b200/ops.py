@@ -145,7 +145,8 @@ def rotate_volume_grad_R(vol: torch.Tensor, grad_out: torch.Tensor, R: torch.Ten
 def score_train(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tensor, W1: torch.Tensor, W2: torch.Tensor,
                 b2: torch.Tensor, workspace: torch.Tensor | None = None):
     """ahv_score_train: the training forward - scores [B,N] from the tensor-core kernel, plus what the backward pass
-    wants back: conv1's ReLU'd output of every item (fp16 [B*N,64,32], 4 KB per item) and 1/scale per pair [B]."""
+    wants back: conv1's ReLU'd output of every item (fp16 [B*N,64,32], 4 KB per item) and per pair [B] the factor
+    that turns it back into conv1's output (2^e1 / scale: the pair scale and W1's normaliser)."""
     vs, tf, R = _dev(vol_src, "vol_src"), _dev(tgt_feat, "tgt_feat"), _dev(R, "R")
     W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
     B = vs.shape[0]

@@ -56,15 +56,26 @@ enum { AHV_VOL_F32 = 0, AHV_VOL_BF16 = 1 };
  *                 take this path (their staging is exact).  About 2e-4 relative.
  * Normalisation, correlation and selection are fp32 in every mode; trilinear resampling is
  * fp32 except in the f16-gather path.
- * Dynamic range: the tensor-core modes multiply each pair's volume by a power of two that maps
- * max|V| into (b/2, b], b = min(4096, 16384 / largest L1 row norm of W1), and undo it before the
- * bias, so one large voxel pushes the rest of the volume towards fp16's subnormals.  Measured on an
- * NVIDIA B200 (1000 W) against fp64, for a standard-normal volume with outlier voxels up to r times
- * larger (scripts/dynamic_range.py, tests/test_gpu_pair_scale.py), the scores meet their gates as follows:
- *   AHV_MATH_TC, fp32 volumes           1e-3 up to r = 1e8 (9.4e-4 there; 1.7e-2 at 1e9)
- *   AHV_MATH_TC_F16GATHER, fp32 volumes 1e-3 up to r = 3e7 (7.4e-4 there; 1.5e-3 at 1e8)
+ * Weight range: the tensor-core modes pack W1 and W2 as fp16(W * 2^-e), powers of two chosen so that
+ * the largest row L1 norm lies in [4, 8) for W1 and in [1, 2) for W2, and undo them with the pair
+ * scale before the bias.  The scores therefore do not depend on the weights' magnitude: scaling W1,
+ * W2 or b2 by a power of two along the score's symmetries (W1 and b2 together, or W2 and b2) gives
+ * bit-identical scores, and weights far below or above fp16's range (down to 1e-7 times and up to
+ * 2e7 times a default initialisation, entries above 65504 included) meet the gates below at the
+ * errors of the default initialisation (scripts/weight_range.py, tests/test_gpu_weight_range.py).
+ * What fp16 cannot absorb is the spread between W1's rows, which sets the precision of the fp16
+ * conv1 output: one row 2^4 times the others stays within every gate; at 2^6 AHV_MATH_TC (8.8e-4)
+ * and bf16 volumes (1.8e-3) still do and AHV_MATH_TC_F16GATHER (2.1e-3) does not; at 2^8 none does.
+ * Dynamic range: each pair's volume is multiplied by a power of two that maps max|V| into (b/2, b],
+ * b = 32768 / L1n with L1n the normalised W1's largest row L1 norm (so b is in (4096, 8192] for any
+ * W1 and conv1's output stays below 2^15), and undone before the bias, so one large voxel pushes the
+ * rest of the volume towards fp16's subnormals.  Measured on an NVIDIA B200 (1000 W) against fp64,
+ * for a standard-normal volume with outlier voxels up to r times larger (scripts/dynamic_range.py,
+ * tests/test_gpu_pair_scale.py), the scores meet their gates as follows, for any W1 magnitude:
+ *   AHV_MATH_TC, fp32 volumes           1e-3 up to r = 1e8 (4.4e-4 there; 7.5e-3 at 1e9)
+ *   AHV_MATH_TC_F16GATHER, fp32 volumes 1e-3 up to r = 1e8 (6.2e-4 there; 8.2e-3 at 1e9)
  *   bf16 volumes (either tensor-core mode) 2e-3 against the bf16-rounded volume and 1e-2 against the
- *                                       unrounded one up to r = 1e8 (1.5e-3 there; 2.1e-2 at 1e9)
+ *                                       unrounded one up to r = 1e8 (6.0e-4 there; 8.6e-3 at 1e9)
  *   AHV_MATH_FP32                       2e-5 up to r = 3e5; beyond it fp32 rounding of the outlier's
  *                                       share (the reference's fp32 path too) reaches 1e-4 at r = 1e7. */
 enum { AHV_MATH_TC = 0, AHV_MATH_FP32 = 1, AHV_MATH_TC_F16GATHER = 2 };
@@ -143,8 +154,9 @@ AHV_API int ahv_resblock3d(const float* x, const float* conv1_w, const float* co
 
 /* Saved-activation form of the training step (the reference's autograd saves ~420 KB per hypothesis; this saves 4 KB):
  * ahv_score_train = ahv_score with AHV_MATH_TC, fp32 volumes, k = 0, that also keeps conv1's ReLU'd output of every
- * (pair, hypothesis) - h1_saved [B*N][64][32] fp16 in the pair's scaled units - and 1/scale per pair
- * (pair_inv_scale [B]); ahv_score_backward_saved = ahv_score_backward reading them instead of recomputing conv1
+ * (pair, hypothesis) - h1_saved [B*N][64][32] fp16 in the kernel's units (pair scale s, normalised W1) - and per
+ * pair the factor that turns it back into conv1's output, 2^e1 / s (pair_inv_scale [B]; 2^-e1 is W1's normaliser);
+ * ahv_score_backward_saved = ahv_score_backward reading them instead of recomputing conv1
  * (786 k of the backward's 2.4 M FMA per item).  math_mode AHV_MATH_FP32: the remaining contractions in fp32 FFMA;
  * AHV_MATH_TC: dA = dH1 W1 and dW1 = dH1^T A on tcgen05 (fp16 operands under power-of-two scales, fp32 accumulation in
  * TMEM; csrc/ahv_score_bwd_tc.cu).  Workspace: ahv_workspace_bytes(B, N, 1). */

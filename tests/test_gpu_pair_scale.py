@@ -1,8 +1,8 @@
 """GPU (B200): the per-pair power-of-two scale of the tensor-core paths, and the dynamic range of their fp16 operands.
 
 The tensor-core kernels do not score the raw volume: stage_pair_volume (csrc/ahv_tc_common.cuh) multiplies each pair's
-volume by its own power of two, chosen from max|V| and the largest L1 row norm of W1, so that the fp16 operands cannot
-overflow.  The gather warps hand 1/scale to the epilogue through an 8-entry ring indexed by pair; the epilogue undoes
+volume by its own power of two, chosen from max|V| and the largest L1 row norm of the normalised W1, so that the fp16
+operands cannot overflow.  The gather warps hand 1/scale to the epilogue through an 8-entry ring indexed by pair; the epilogue undoes
 the scale before it adds b2, and the training forward writes it out for the tcgen05 backward.  The gather runs several
 tiles ahead of the epilogue, and with N = 1 or 2 every tile starts a new pair.
 
@@ -13,6 +13,8 @@ all get different scales.  References: the AHV_MATH_FP32 kernel (an independent 
 pair, fp64 `oracle.score_torch` for a sample that includes the pairs on CTA boundaries.
 
 The second half bounds the outlier-to-bulk ratio each mode handles (the numbers quoted in include/ahv_b200.h)."""
+import math
+
 import numpy as np
 import pytest
 import torch
@@ -139,18 +141,30 @@ def test_mixed_scales_every_mode(ahv, golden, oracle, B, N, per_pair, voldt):
             assert torch.equal(alone.scores[0], s[b]), (mode, b)
 
 
+def _w1_normaliser(W1):
+    """2^e1, e1 = floor(log2 of W1's largest row L1 norm) - 2: the tensor-core kernels pack W1 * 2^-e1, whose largest
+    row L1 norm lies in [4, 8)."""
+    return 2.0 ** (math.floor(math.log2(float(W1.double().abs().sum(1).max()))) - 2)
+
+
 def _scale_bound(W1):
-    """stage_pair_volume's target for max|V| * scale: min(4096, 16384 / largest L1 row norm of W1)."""
-    l1max = float(W1.float().abs().sum(1).max())
-    return min(4096.0, 16384.0 / l1max)
+    """stage_pair_volume's target for max|V| * scale: 32768 / (largest L1 row norm of the normalised W1, in [4, 8)),
+    capped at 8192 - so in (4096, 8192] whatever W1's magnitude."""
+    l1max = float(W1.double().abs().sum(1).max()) / _w1_normaliser(W1)
+    assert 4.0 <= l1max < 8.0
+    return min(8192.0, 32768.0 / l1max)
 
 
+@pytest.mark.parametrize("w1_exp", [0, -12, 12])
 @pytest.mark.parametrize("B,N,per_pair", [(300, 1, False), (97, 2, True), (40, 3, True), (160, 7, False)])
-def test_training_forward_keeps_each_pairs_scale(ahv, golden, B, N, per_pair):
-    """ahv_score_train's 1/scale per pair is the exact power of two of the scale rule for that pair's own max|V|; it,
-    the kept conv1 activations and the scores do not depend on the rest of the batch, and the scores are those of the
-    inference kernel."""
+def test_training_forward_keeps_each_pairs_scale_at_every_weight_magnitude(ahv, golden, B, N, per_pair, w1_exp):
+    """ahv_score_train's pair_inv is 2^e1 / scale with the exact power of two of the scale rule for that pair's own
+    max|V| (2^e1: W1's normaliser), for the golden W1 and for W1 scaled by 1.37 * 2^-12 and 1.37 * 2^12 (the rule, and
+    so max|V| * scale, does not depend on W1's magnitude); pair_inv, the kept conv1 activations and the scores do not
+    depend on the rest of the batch, and the scores are those of the inference kernel."""
     W1, W2, b2 = _weights(golden)
+    if w1_exp:
+        W1 = W1 * (1.37 * 2.0 ** w1_exp)
     vs, vt = (t.to(DEV) for t in _mixed_batch(B, seed=7 * B + N))
     R = _rotations(ahv, B, N, per_pair, seed=3 * B + N)
     tgt = ahv.ops.forward_3d2d(vt, W1, W2, b2)
@@ -158,7 +172,7 @@ def test_training_forward_keeps_each_pairs_scale(ahv, golden, B, N, per_pair):
     mant, _ = torch.frexp(pinv)
     assert bool((mant == 0.5).all()), pinv[mant != 0.5]
     bound = _scale_bound(W1)
-    ratio = vs.abs().flatten(1).max(1).values.double() / pinv.double()   # max|V| * scale, exact
+    ratio = vs.abs().flatten(1).max(1).values.double() * _w1_normaliser(W1) / pinv.double()   # max|V| * scale, exact
     assert bool(((ratio > bound / 2) & (ratio <= bound)).all()), (bound, ratio[(ratio <= bound / 2) | (ratio > bound)])
     # neighbouring pairs (and pairs 8 apart) really do differ in scale, or this test could not see a mix-up
     assert bool((pinv[1:] != pinv[:-1]).all()) and bool((pinv[8:] != pinv[:-8]).all())
@@ -213,11 +227,11 @@ def test_saved_activation_backward_on_mixed_scales(ahv, golden, oracle, per_pair
 # ---- dynamic range of the fp16 operands --------------------------------------------------------------------------
 # Outlier-to-bulk ratio r = the largest |outlier| over the bulk's standard deviation.  Each pair of a standard-normal
 # bulk carries two outliers, +r/3 and -r (r = 3e4: the 1e4 and -3e4 of a trained checkpoint's heavy tail), one of
-# them on a corner voxel.  With the golden head the pair scale maps r into (2^9.6, 2^10.6], so the bulk nears fp16's
-# smallest normal, 2^-14, around r = 1e7.  scripts/dynamic_range.py sweeps r up to 1e9 on the same inputs; the largest
+# them on a corner voxel.  With the golden head the pair scale maps r into (2^11.6, 2^12.6], so the bulk nears fp16's
+# smallest normal, 2^-14, around r = 3e7.  scripts/dynamic_range.py sweeps r up to 1e9 on the same inputs; the largest
 # r at which each mode met its gate there is MAX_RATIO (include/ahv_b200.h quotes it), and every mode is tested up to it.
 RATIOS = [1e2, 1e3, 1e4, 3e4, 1e5, 3e5, 1e6, 1e7, 3e7, 1e8]
-MAX_RATIO = {"fp32": 3e5, "tc": 1e8, "f16gather": 3e7, "bf16": 1e8}
+MAX_RATIO = {"fp32": 3e5, "tc": 1e8, "f16gather": 1e8, "bf16": 1e8}
 
 
 def _outlier_volumes(B, r, seed):
