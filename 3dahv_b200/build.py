@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "lib3dahv_b200.so")
-SOURCES = ["ahv_api.cu", "ahv_so3.cu", "ahv_score_fp32.cu", "ahv_score_bwd.cu", "ahv_ascent.cu", "ahv_score_bwd_tc.cu", "ahv_score_tc.cu", "ahv_topk.cu", "ahv_diag.cu", "ahv_exchange.cu", "ahv_lift.cu", "ahv_infonce.cu"]
+SOURCES = ["ahv_api.cu", "ahv_so3.cu", "ahv_score_fp32.cu", "ahv_score_bwd.cu", "ahv_ascent.cu", "ahv_score_bwd_tc.cu", "ahv_score_tc.cu", "ahv_topk.cu", "ahv_topk_distinct.cu", "ahv_diag.cu", "ahv_exchange.cu", "ahv_lift.cu", "ahv_infonce.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-std=c++17", "-lineinfo", "--fmad=true",

@@ -360,13 +360,17 @@ AHV_API size_t ahv_refine_gradient_workspace_bytes(int B, int64_t N, int k) {
          align_up(topk_workspace_bytes(B, k, 1), 256);
 }
 
-AHV_API int ahv_refine_gradient(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
-                                const float* W1, const float* W2, const float* b2, const float* base, int k, int steps,
-                                float step_deg, float* first_val, int64_t* first_idx, float* first_R, float* R_all,
-                                float* score_all, float* best_val, int64_t* best_idx, float* R_best, int B, int64_t N,
-                                int math_mode, void* workspace, size_t workspace_bytes, void* stream) {
+namespace {
+bool min_sep_ok(float min_sep_deg) { return std::isfinite(min_sep_deg) && min_sep_deg >= 0.0f && min_sep_deg <= 180.0f; }
+
+// ahv_refine_gradient (min_sep_deg == 0) and ahv_refine_gradient_distinct: the same chain apart from its first pass
+int refine_gradient(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair, const float* W1,
+                    const float* W2, const float* b2, const float* base, int k, int steps, float step_deg, float min_sep_deg,
+                    float* first_val, int64_t* first_idx, float* first_R, float* R_all, float* score_all, float* best_val,
+                    int64_t* best_idx, float* R_best, int B, int64_t N, int math_mode, void* workspace,
+                    size_t workspace_bytes, void* stream) {
   if (B < 1 || N < 1 || N > 0x7fffffffLL || k < 1 || k > kMaxK || k > N) return AHV_EINVAL;
-  if (!ascent_args_ok(vol_dtype, steps, step_deg)) return AHV_EINVAL;
+  if (!ascent_args_ok(vol_dtype, steps, step_deg) || !min_sep_ok(min_sep_deg)) return AHV_EINVAL;
   if (math_mode != AHV_MATH_TC && math_mode != AHV_MATH_FP32 && math_mode != AHV_MATH_TC_F16GATHER) return AHV_EINVAL;
   if (!vol_src || !vol_tgt || !R || !W1 || !W2 || !b2 || !base || !first_val || !first_idx || !first_R || !R_all ||
       !score_all || !best_val || !best_idx || !workspace)
@@ -382,19 +386,68 @@ AHV_API int ahv_refine_gradient(const void* vol_src, int vol_dtype, const float*
   cudaStream_t s = (cudaStream_t)stream;
   unsigned char* ws = static_cast<unsigned char*>(workspace);
   float* tgt = reinterpret_cast<float*>(ws + ws1);
-  // pass 1: the whole set, top-k and their rotations
-  st = ahv_verify(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, first_val, first_idx, first_R, k, 0,
-                  B, N, math_mode, ws, ws1, stream);
-  if (st != AHV_OK) return st;
+  const bool distinct = min_sep_deg > 0.0f;
+  if (!distinct) {
+    // pass 1: the whole set, top-k and their rotations
+    st = ahv_verify(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, first_val, first_idx, first_R, k,
+                    0, B, N, math_mode, ws, ws1, stream);
+    if (st != AHV_OK) return st;
+  }
   // the ascent scores in fp32 against fp32 target features (bit-equal to ahv_forward_3d2d), whatever math_mode is
   st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
   if (st != AHV_OK) return st;
-  st = launch_gradient_ascent(vol_src, vol_dtype, tgt, first_R, W1, W2, b2, base, steps, step_deg, R_all, score_all, B, k, s);
+  if (distinct) {
+    // pass 1: every score of the set (the fused k = 1 arg-max writes none), then the k distinct winners
+    st = ahv_score(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, nullptr, nullptr, nullptr, 0, 0, B, N,
+                   math_mode, ws, ws1, stream);
+    if (st != AHV_OK) return st;
+    st = launch_topk_distinct(reinterpret_cast<const float*>(ws), R, r_per_pair != 0, B, N, k, min_sep_deg, first_val,
+                              first_idx, first_R, s);
+    if (st != AHV_OK) return st;
+  }
+  // empty slots (fewer than k distinct winners) are not ascended: R_all NaN, score_all -inf
+  st = launch_gradient_ascent(vol_src, vol_dtype, tgt, first_R, W1, W2, b2, base, steps, step_deg, R_all, score_all, B, k, s,
+                              distinct ? first_idx : nullptr);
   if (st != AHV_OK) return st;
   // per-pair arg-max over the k ascended candidates
   st = launch_topk(score_all, B, k, 1, 0, best_val, best_idx, ws + ws1 + ws_tgt, ws_top, s);
   if (st != AHV_OK || !R_best) return st;
   return launch_gather_rotations(R_all, 1, best_idx, 0, B, k, 1, R_best, s);
+}
+}  // namespace
+
+AHV_API int ahv_refine_gradient(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
+                                const float* W1, const float* W2, const float* b2, const float* base, int k, int steps,
+                                float step_deg, float* first_val, int64_t* first_idx, float* first_R, float* R_all,
+                                float* score_all, float* best_val, int64_t* best_idx, float* R_best, int B, int64_t N,
+                                int math_mode, void* workspace, size_t workspace_bytes, void* stream) {
+  return refine_gradient(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, 0.0f, first_val,
+                         first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode, workspace,
+                         workspace_bytes, stream);
+}
+
+AHV_API int ahv_refine_gradient_distinct(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R,
+                                         int r_per_pair, const float* W1, const float* W2, const float* b2, const float* base,
+                                         int k, int steps, float step_deg, float min_sep_deg, float* first_val,
+                                         int64_t* first_idx, float* first_R, float* R_all, float* score_all, float* best_val,
+                                         int64_t* best_idx, float* R_best, int B, int64_t N, int math_mode, void* workspace,
+                                         size_t workspace_bytes, void* stream) {
+  return refine_gradient(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, min_sep_deg,
+                         first_val, first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode,
+                         workspace, workspace_bytes, stream);
+}
+
+// ---- top-k of distinct rotations: greedy geodesic non-maximum suppression on SO(3) (extension) ------------
+AHV_API int ahv_topk_distinct(const float* scores, const float* R, int r_per_pair, int B, int64_t N, int k,
+                              float min_sep_deg, float* topk_val, int64_t* topk_idx, float* R_best, void* stream) {
+  if (B < 0 || N < 0 || N > 0x7fffffffLL || k < 1 || k > kMaxK || !min_sep_ok(min_sep_deg)) return AHV_EINVAL;
+  if (B > 0 && (!topk_val || !topk_idx)) return AHV_EINVAL;
+  if ((int64_t)B * N > 0 && (!scores || !R)) return AHV_EINVAL;
+  if (!aligned16(R) || !aligned16(R_best)) return AHV_EINVAL;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  return launch_topk_distinct(scores, R, r_per_pair != 0, B, N, k, min_sep_deg, topk_val, topk_idx, R_best,
+                              (cudaStream_t)stream);
 }
 
 // ---- hypothesis set sharded over the GPUs of one node: winners exchanged through peer memory -------------

@@ -72,7 +72,7 @@ __global__ void __launch_bounds__(kThreads, 1)
 ascent_fp32_kernel(const T* __restrict__ vol_src, const float* __restrict__ tgt_feat, const float* __restrict__ R_init,
                    const float* __restrict__ W1, const float* __restrict__ W2, const float* __restrict__ b2,
                    const float* __restrict__ base, int steps, float theta0, float* __restrict__ R_out,
-                   float* __restrict__ score_out, int B, int K) {
+                   float* __restrict__ score_out, int B, int K, const int64_t* __restrict__ skip_idx) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   AscentSmem& as = *reinterpret_cast<AscentSmem*>(smem_raw);
   Fp32Smem& sm = as.f;
@@ -89,6 +89,11 @@ ascent_fp32_kernel(const T* __restrict__ vol_src, const float* __restrict__ tgt_
   for (int64_t it = lo; it < hi; ++it) {
     const int b = (int)(it / K);
     __syncthreads();  // the previous item is done with the volume, R and Rcur
+    if (skip_idx && skip_idx[it] < 0) {  // an empty selection slot (ahv_refine_gradient_distinct): nothing to ascend
+      if (t < 9) R_out[(size_t)it * 9 + t] = nanf("");
+      if (t == 0) score_out[it] = -INFINITY;
+      continue;
+    }
     if (b != cur_b) {
       stage_volume<T>(sm.vol, vol_src + (size_t)b * kC * kVox);
 #pragma unroll
@@ -144,7 +149,7 @@ ascent_fp32_kernel(const T* __restrict__ vol_src, const float* __restrict__ tgt_
 
 int launch_gradient_ascent(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R_init, const float* W1,
                            const float* W2, const float* b2, const float* base, int steps, float step_deg, float* R_out,
-                           float* score_out, int B, int K, cudaStream_t s) {
+                           float* score_out, int B, int K, cudaStream_t s, const int64_t* skip_idx) {
   const int64_t total = (int64_t)B * K;
   if (total == 0) return AHV_OK;
   int dev = 0, sms = 0;
@@ -156,11 +161,11 @@ int launch_gradient_ascent(const void* vol_src, int vol_dtype, const float* tgt_
   if (vol_dtype == AHV_VOL_F32) {
     AHV_CUDA_OK(cudaFuncSetAttribute(ascent_fp32_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ascent_fp32_kernel<float><<<grid, kThreads, smem, s>>>((const float*)vol_src, tgt_feat, R_init, W1, W2, b2, base, steps,
-                                                           theta0, R_out, score_out, B, K);
+                                                           theta0, R_out, score_out, B, K, skip_idx);
   } else {
     AHV_CUDA_OK(cudaFuncSetAttribute(ascent_fp32_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ascent_fp32_kernel<__nv_bfloat16><<<grid, kThreads, smem, s>>>((const __nv_bfloat16*)vol_src, tgt_feat, R_init, W1, W2,
-                                                                   b2, base, steps, theta0, R_out, score_out, B, K);
+                                                                   b2, base, steps, theta0, R_out, score_out, B, K, skip_idx);
   }
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;

@@ -153,7 +153,7 @@ int launch_infonce(const float* scores, const float* R, int r_per_pair, const fl
                    float* loss, float* grad, int B, int64_t N, cudaStream_t s);
 int launch_gradient_ascent(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R_init, const float* W1,
                            const float* W2, const float* b2, const float* base, int steps, float step_deg, float* R_out,
-                           float* score_out, int B, int K, cudaStream_t s);
+                           float* score_out, int B, int K, cudaStream_t s, const int64_t* skip_idx = nullptr);
 int launch_forward_3d2d(const float* vol, const float* W1, const float* W2, const float* b2,
                         float* feat, int64_t m, cudaStream_t s);
 int launch_tgt_feat(const float* vol_tgt, const float* W1, const float* W2, const float* b2,
@@ -182,5 +182,7 @@ int launch_topk_merge(const float* vals, const int64_t* idx, int parts, int B, i
                       int64_t* out_idx, cudaStream_t s);
 int launch_gather_rotations(const float* R, int r_per_pair, const int64_t* idx, int64_t idx_offset,
                             int B, int64_t N, int k, float* R_out, cudaStream_t s);
+int launch_topk_distinct(const float* scores, const float* R, int r_per_pair, int B, int64_t N, int k, float min_sep_deg,
+                         float* val, int64_t* idx, float* R_best, cudaStream_t s);
 
 }  // namespace ahv

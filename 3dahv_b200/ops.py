@@ -456,9 +456,11 @@ def gradient_ascent(vol_src, tgt_feat, R_init, W1, W2, b2, steps: int = 20, step
 
 
 def refine_gradient(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, steps: int = 20, step_deg: float = 1.0, math: int = MATH_TC,
-                    workspace: torch.Tensor | None = None, out=None):
+                    workspace: torch.Tensor | None = None, out=None, min_sep_deg: float = 0.0):
     """ahv_refine_gradient: top-k over the set, gradient ascent of the fp32 score from each winner, per-pair arg-max -
     one C call, no torch ops, CUDA-graph capturable (pass `out` = the tuple a previous call returned to reuse its buffers).
+    min_sep_deg > 0 calls ahv_refine_gradient_distinct: the first pass keeps the k winners of `topk_distinct` instead, and
+    its empty slots come back as first_idx -1, R_all NaN, score_all -inf.
     Returns (first_val [B,k], first_idx [B,k], first_R [B,k,3,3], R_all [B,k,3,3], score_all [B,k], best_val [B],
     best_idx [B], R_best [B,3,3], workspace)."""
     vs, vdt = _vol_src(vol_src)
@@ -482,12 +484,15 @@ def refine_gradient(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, steps: int = 2
     if workspace is None or workspace.numel() * workspace.element_size() < need:
         workspace = torch.empty(max(need, 16), device=dev, dtype=torch.uint8)
     base = base_coords(dev)
+    head = (vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
+            base.data_ptr(), k, int(steps), float(step_deg))
+    tail = (fv.data_ptr(), fi.data_ptr(), fR.data_ptr(), Ra.data_ptr(), sa.data_ptr(), bv.data_ptr(), bi.data_ptr(), bR.data_ptr(),
+            B, N, math, workspace.data_ptr(), workspace.numel() * workspace.element_size(), _stream(vs))
     with torch.cuda.device(dev):
-        _lib.check(_lib.lib().ahv_refine_gradient(
-            vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
-            base.data_ptr(), k, int(steps), float(step_deg), fv.data_ptr(), fi.data_ptr(), fR.data_ptr(), Ra.data_ptr(),
-            sa.data_ptr(), bv.data_ptr(), bi.data_ptr(), bR.data_ptr(), B, N, math, workspace.data_ptr(),
-            workspace.numel() * workspace.element_size(), _stream(vs)), "ahv_refine_gradient")
+        if min_sep_deg == 0:
+            _lib.check(_lib.lib().ahv_refine_gradient(*head, *tail), "ahv_refine_gradient")
+        else:
+            _lib.check(_lib.lib().ahv_refine_gradient_distinct(*head, float(min_sep_deg), *tail), "ahv_refine_gradient_distinct")
     return fv, fi, fR, Ra, sa, bv, bi, bR, workspace
 
 
@@ -561,6 +566,28 @@ def topk(scores: torch.Tensor, k: int, idx_offset: int = 0):
         st = _lib.lib().ahv_topk(s.data_ptr(), B, N, k, idx_offset, val.data_ptr(), idx.data_ptr(), ws.data_ptr(), ws.numel(), _stream(s))
     _lib.check(st, "ahv_topk")
     return val, idx
+
+
+def topk_distinct(scores: torch.Tensor, R: torch.Tensor, k: int, min_sep_deg: float, gather: bool = True):
+    """ahv_topk_distinct: per pair, the k best hypotheses whose rotations lie pairwise more than `min_sep_deg` apart
+    (greedy geodesic non-maximum suppression in `topk`'s order).  scores [B,N]; R [N,3,3] or [B,N,3,3].  Returns
+    (topk_val [B,k], topk_idx [B,k], R_best [B,k,3,3] or None); slots no hypothesis fills are (-inf, -1, NaN).
+    min_sep_deg = 0 gives `topk` bit for bit, 180 the top-1 alone."""
+    s, R = _dev(scores, "scores"), _dev(R, "R")
+    B, N = s.shape
+    per_pair = R.dim() == 4
+    if tuple(R.shape) != ((B, N, 3, 3) if per_pair else (N, 3, 3)):
+        raise ValueError("R must be [N,3,3] or [B,N,3,3] for scores [B,N]")
+    if not 1 <= k <= 32:
+        raise ValueError("k must be in [1,32]")
+    val = torch.empty(B, k, device=s.device, dtype=torch.float32)
+    idx = torch.empty(B, k, device=s.device, dtype=torch.int64)
+    Rb = torch.empty(B, k, 3, 3, device=s.device, dtype=torch.float32) if gather else None
+    with torch.cuda.device(s.device):
+        st = _lib.lib().ahv_topk_distinct(s.data_ptr(), R.data_ptr(), int(per_pair), B, N, k, float(min_sep_deg), val.data_ptr(),
+                                          idx.data_ptr(), Rb.data_ptr() if gather else None, _stream(s))
+    _lib.check(st, "ahv_topk_distinct")
+    return val, idx, Rb
 
 
 def topk_merge(vals: torch.Tensor, idx: torch.Tensor):

@@ -68,8 +68,9 @@ class HypothesisVerifier:
 
     @torch.no_grad()
     def score(self, vol_src, vol_tgt, R, k: int = 1, return_scores: bool = True, tgt_feat=None,
-              idx_offset: int = 0, gather: bool = True) -> VerifyResult:
-        """vol_src/vol_tgt [B,16,8,8,8]; R [N,3,3] shared or [B,N,3,3] per pair."""
+              idx_offset: int = 0, gather: bool = True, min_sep_deg: float = 0.0) -> VerifyResult:
+        """vol_src/vol_tgt [B,16,8,8,8]; R [N,3,3] shared or [B,N,3,3] per pair.  min_sep_deg > 0 keeps the k best
+        rotations that lie pairwise more than min_sep_deg apart (`ops.topk_distinct`; empty slots are -inf / -1 / NaN)."""
         dev = vol_src.device
         W1, W2, b2 = self._weights_on(dev)
         per_pair = R.dim() == 4
@@ -80,6 +81,13 @@ class HypothesisVerifier:
         k = min(k, N)
         vs = vol_src if vol_src.dtype == torch.bfloat16 else vol_src.float()
         ws = self._workspace(B, N, k, dev)
+        if min_sep_deg > 0:   # greedy NMS does not compose from per-shard lists: no idx_offset
+            if idx_offset:
+                raise ValueError("min_sep_deg > 0 selects over the whole set: idx_offset must be 0")
+            tf = self.target_features(vol_tgt) if tgt_feat is None else tgt_feat
+            scores = ops.score(vs, tf, R, W1, W2, b2, k=0, math=self.math, workspace=ws)[0]
+            val, idx, R_best = ops.topk_distinct(scores, R, k, min_sep_deg, gather=gather)
+            return VerifyResult(scores if return_scores else None, val, idx, R_best)
         if tgt_feat is None:   # one C call for the whole step (2 launches when k == 1)
             scores, val, idx, R_best = ops.verify(vs, vol_tgt.float(), R, W1, W2, b2, k=k, idx_offset=idx_offset,
                                                   math=self.math, return_scores=return_scores, gather=gather,
@@ -169,16 +177,19 @@ class HypothesisVerifier:
         return ops.gather_rotations(R_all, idx)[:, 0], val[:, 0], R_all, s_all
 
     @torch.no_grad()
-    def refine_by_gradient(self, vol_src, vol_tgt, R, k: int = 32, steps: int = 20, step_deg: float = 1.0):
+    def refine_by_gradient(self, vol_src, vol_tgt, R, k: int = 32, steps: int = 20, step_deg: float = 1.0,
+                           min_sep_deg: float = 0.0):
         """Grid pass + gradient ascent in one C call (`ahv_refine_gradient`; BASELINE config 4's accurate path): score
         the set with this verifier's math mode, keep the top-k, run `ascend` from each winner, return the best.
+        min_sep_deg > 0 keeps the top-k of rotations pairwise more than min_sep_deg apart instead
+        (`ahv_refine_gradient_distinct`), so the ascents start in distinct basins; slots left empty are not ascended.
         Returns (R_best [B,3,3], score [B], first pass as a VerifyResult, R_all [B,k,3,3], score_all [B,k])."""
         W1, W2, b2 = self._weights_on(vol_src.device)
         k = min(k, R.shape[1] if R.dim() == 4 else R.shape[0])
         vs = vol_src if vol_src.dtype == torch.bfloat16 else vol_src.float()
         fv, fi, fR, Ra, sa, bv, bi, bR, self._ws_refine_gradient = ops.refine_gradient(
             vs, vol_tgt.float(), R, W1, W2, b2, k=k, steps=steps, step_deg=step_deg, math=self.math,
-            workspace=getattr(self, "_ws_refine_gradient", None))
+            workspace=getattr(self, "_ws_refine_gradient", None), min_sep_deg=min_sep_deg)
         return bR, bv, VerifyResult(None, fv, fi, fR), Ra, sa
 
 
@@ -251,14 +262,17 @@ class GraphedRefiner:
     arg-max; BASELINE config 4) for fixed (B, N, k, m): the whole chain - target features, both scoring passes, top-k,
     candidate generation, selection - is one C call with no host step or torch op inside, so it captures as it stands.
     method="gradient" captures `ahv_refine_gradient` instead (dense set -> top-k -> `steps` steps of gradient ascent
-    from each winner, starting at step_deg -> arg-max; m, max_angle_deg and seed are unused).
+    from each winner, starting at step_deg -> arg-max; m, max_angle_deg and seed are unused), or with min_sep_deg > 0
+    `ahv_refine_gradient_distinct` (the top-k of rotations pairwise more than min_sep_deg apart).
     Outputs are static tensors valid until the next replay."""
 
     def __init__(self, verifier: HypothesisVerifier, B: int, N: int, k: int = 32, m: int = 64, max_angle_deg: float = 5.0,
                  seed: int = 0, device="cuda", vol_dtype=torch.float32, method: str = "perturb", steps: int = 20,
-                 step_deg: float = 1.0):
+                 step_deg: float = 1.0, min_sep_deg: float = 0.0):
         if method not in ("perturb", "gradient"):
             raise ValueError('method must be "perturb" or "gradient"')
+        if min_sep_deg != 0 and method != "gradient":
+            raise ValueError('min_sep_deg applies to method="gradient" only')
         dev = torch.device(device)
         self.v = verifier.to(dev)
         self.vol_src = torch.zeros(B, 16, 8, 8, 8, device=dev, dtype=vol_dtype)
@@ -270,7 +284,7 @@ class GraphedRefiner:
         def run(out=None, ws=None):
             if method == "gradient":
                 return ops.refine_gradient(self.vol_src, self.vol_tgt, self.R, W1, W2, b2, k=k, steps=steps, step_deg=step_deg,
-                                           math=self.v.math, workspace=ws, out=out)
+                                           math=self.v.math, workspace=ws, out=out, min_sep_deg=min_sep_deg)
             return ops.refine(self.vol_src, self.vol_tgt, self.R, W1, W2, b2, k=k, m=m, max_angle_deg=max_angle_deg, seed=seed,
                               math=self.v.math, workspace=ws, out=out)
 

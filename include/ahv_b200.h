@@ -265,6 +265,32 @@ AHV_API int ahv_refine_gradient(const void* vol_src, int vol_dtype, const float*
                                 float* score_all, float* best_val, int64_t* best_idx, float* R_best, int B, int64_t N,
                                 int math_mode, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ahv_refine_gradient that ascends from k DISTINCT basins (extension): the grid pass scores the whole set (target
+ * features, then ahv_score with k = 0; no fused arg-max, whose scores are never written) and keeps the k winners of
+ * ahv_topk_distinct(min_sep_deg) in first_val/idx/R.  Slots left empty there (fewer than k rotations pairwise more than
+ * min_sep_deg apart) are not ascended: R_all NaN, score_all -inf, so the arg-max never picks one.  0 <= min_sep_deg
+ * <= 180; with min_sep_deg == 0 every output equals ahv_refine_gradient's bit for bit.  Every other argument, rule and
+ * the workspace (ahv_refine_gradient_workspace_bytes) are ahv_refine_gradient's. */
+AHV_API int ahv_refine_gradient_distinct(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R,
+                                         int r_per_pair, const float* W1, const float* W2, const float* b2, const float* base,
+                                         int k, int steps, float step_deg, float min_sep_deg, float* first_val,
+                                         int64_t* first_idx, float* first_R, float* R_all, float* score_all, float* best_val,
+                                         int64_t* best_idx, float* R_best, int B, int64_t N, int math_mode, void* workspace,
+                                         size_t workspace_bytes, void* stream);
+
+/* Top-k of distinct rotations (extension): greedy geodesic non-maximum suppression on SO(3) over the score-sorted
+ * hypotheses of each pair.  With key(n) = ahv_topk's order (score descending, ties -> lowest index, NaN as ahv_topk
+ * orders it), t(a,b) = trace(R_a R_b^T) in fp32 (nine individually rounded products summed left to right, no FMA) and
+ * c = fp32(1 + 2 cos(min_sep_deg * pi / 180)) evaluated in double:
+ *   w_0 = the largest key;  w_j = the largest key(n) < key(w_{j-1}) with t(n, w_i) < c for every i < j,
+ * stopping at k winners or when none qualifies; the later slots are empty (value -inf, index -1, rotation NaN).
+ * min_sep_deg == 0 suppresses nothing (the result is ahv_topk's bit for bit); min_sep_deg == 180 keeps the top-1 alone.
+ * scores [B,N]; R [N,3,3] (r_per_pair == 0) or [B,N,3,3]; topk_val [B,k], topk_idx [B,k] int64, R_best [B,k,3,3] or
+ * NULL.  1 <= k <= 32, 0 <= min_sep_deg <= 180, N <= 2^31 - 1; R and R_best 16-byte aligned.  One launch (a cluster of
+ * 8 CTAs per pair), no workspace, no allocation, no host synchronisation: deterministic and CUDA-graph capturable. */
+AHV_API int ahv_topk_distinct(const float* scores, const float* R, int r_per_pair, int B, int64_t N, int k,
+                              float min_sep_deg, float* topk_val, int64_t* topk_idx, float* R_best, void* stream);
+
 /* torch.max / top-k over an existing score matrix (modules/model.py:195). */
 AHV_API int ahv_topk(const float* scores, int B, int64_t N, int k, int64_t idx_offset, float* topk_val,
              int64_t* topk_idx, void* workspace, size_t workspace_bytes, void* stream);
