@@ -11,6 +11,14 @@ using namespace ahv;
 namespace {
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+template <class... P> bool all_aligned16(P... p) { return (aligned16(p) && ...); }
+template <class... P> bool all_set(P... p) { return (... && (p != nullptr)); }
+
+// Argument rules shared by the entries (each entry keeps its own order of checks).
+bool vol_dtype_ok(int vol_dtype) { return vol_dtype == AHV_VOL_F32 || vol_dtype == AHV_VOL_BF16; }
+bool math_mode_ok(int m) { return m == AHV_MATH_TC || m == AHV_MATH_FP32 || m == AHV_MATH_TC_F16GATHER; }
+bool n_ok(int64_t N) { return N >= 0 && N <= 0x7fffffffLL; }  // hypotheses per pair: 31-bit indices
+bool k_ok(int k) { return k >= 1 && k <= kMaxK; }
 
 // The library contains sm_100a code only; refuse anything else loudly.
 int check_device() {
@@ -22,6 +30,34 @@ int check_device() {
 }
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// Workspace layouts: the offset of each region (each 256-byte aligned) and the size of the whole.
+// The verification workspace: [scores B*N fp32 | top-k partials | tensor-core scratch | per-shard top-k lists].
+// ahv_score needs the bytes up to `lists` only.
+struct VerifyWs {
+  size_t topk, tc, lists, total;
+  VerifyWs(int B, int64_t N, int k)
+      : topk(align_up((size_t)B * (size_t)N * sizeof(float), 256)),
+        tc(topk + align_up(topk_workspace_bytes(B, N, k), 256)),
+        lists(tc + align_up(score_tc_workspace_bytes(B, N), 256)),
+        total(lists + align_up((size_t)B * (size_t)(k > 0 ? k : 1) * (sizeof(float) + sizeof(int64_t)), 256)) {}
+};
+
+// ahv_refine: [the grid pass's verification workspace | the candidate pass's ([B, k*m], arg-max)]
+struct RefineWs {
+  size_t cand, total;
+  RefineWs(int B, int64_t N, int k, int m)
+      : cand(VerifyWs(B, N, k).total), total(cand + VerifyWs(B, (int64_t)k * m, 1).total) {}
+};
+
+// ahv_refine_gradient: [the grid pass's verification workspace | target features B*32*64 fp32 | top-k partials over [B,k]]
+struct RefineGradientWs {
+  size_t tgt, top, total;
+  RefineGradientWs(int B, int64_t N, int k)
+      : tgt(VerifyWs(B, N, k).total),
+        top(tgt + align_up((size_t)B * kO * kP * sizeof(float), 256)),
+        total(top + align_up(topk_workspace_bytes(B, k, 1), 256)) {}
+};
 
 }  // namespace
 
@@ -90,9 +126,9 @@ AHV_API int ahv_score_backward(const float* vol_src, const float* tgt_feat, cons
                                const float* W1, const float* W2, const float* b2, const float* base,
                                const float* grad_scores, float* grad_vol, float* grad_tgt, float* grad_W1,
                                float* grad_W2, float* grad_b2, int B, int64_t N, void* stream) {
-  if (B < 0 || N < 0 || N > 0x7fffffffLL) return AHV_EINVAL;
-  if ((int64_t)B * N > 0 && (!vol_src || !tgt_feat || !R || !W1 || !W2 || !b2 || !base || !grad_scores || !grad_vol ||
-                             !grad_tgt || !grad_W1 || !grad_W2 || !grad_b2))
+  if (B < 0 || !n_ok(N)) return AHV_EINVAL;
+  if ((int64_t)B * N > 0 &&
+      !all_set(vol_src, tgt_feat, R, W1, W2, b2, base, grad_scores, grad_vol, grad_tgt, grad_W1, grad_W2, grad_b2))
     return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
@@ -113,11 +149,10 @@ AHV_API int ahv_score_backward_ex(const float* vol_src, const float* tgt_feat, c
                                   const float* grad_scores, const void* h1_saved, const float* pair_inv_scale,
                                   float* grad_vol, float* grad_tgt, float* grad_W1, float* grad_W2, float* grad_b2,
                                   float* grad_R, int B, int64_t N, void* stream) {
-  if (B < 0 || N < 0 || N > 0x7fffffffLL) return AHV_EINVAL;
+  if (B < 0 || !n_ok(N)) return AHV_EINVAL;
   if (!grad_vol && !grad_tgt && !grad_W1 && !grad_W2 && !grad_b2 && !grad_R) return AHV_EINVAL;
   if (!h1_saved != !pair_inv_scale || !aligned16(h1_saved)) return AHV_EINVAL;
-  if ((int64_t)B * N > 0 && (!vol_src || !tgt_feat || !R || !W1 || !W2 || !b2 || !base || !grad_scores))
-    return AHV_EINVAL;
+  if ((int64_t)B * N > 0 && !all_set(vol_src, tgt_feat, R, W1, W2, b2, base, grad_scores)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
   return launch_score_bwd(vol_src, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, grad_scores, grad_vol, grad_tgt,
@@ -136,7 +171,7 @@ AHV_API int ahv_infonce(const float* scores, const float* R, int r_per_pair, con
 AHV_API int ahv_resblock3d(const float* x, const float* conv1_w, const float* conv2_w, const float* down_w, float* out,
                            int64_t m, void* stream) {
   if (m < 0 || (m > 0 && (!x || !conv1_w || !conv2_w || !down_w || !out))) return AHV_EINVAL;
-  if (!aligned16(x) || !aligned16(out)) return AHV_EINVAL;
+  if (!all_aligned16(x, out)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
   return launch_resblock3d(x, conv1_w, conv2_w, down_w, out, m, (cudaStream_t)stream);
@@ -146,13 +181,10 @@ AHV_API int ahv_score_train(const float* vol_src, const float* tgt_feat, const f
                             const float* W2, const float* b2, const float* base, float* scores, void* h1_saved,
                             float* pair_inv_scale, int B, int64_t N, void* workspace, size_t workspace_bytes,
                             void* stream) {
-  if (B < 0 || N < 0 || N > 0x7fffffffLL) return AHV_EINVAL;
-  if ((int64_t)B * N > 0 && (!vol_src || !tgt_feat || !R || !W1 || !W2 || !b2 || !base || !scores || !h1_saved ||
-                             !pair_inv_scale || !workspace))
+  if (B < 0 || !n_ok(N)) return AHV_EINVAL;
+  if ((int64_t)B * N > 0 && !all_set(vol_src, tgt_feat, R, W1, W2, b2, base, scores, h1_saved, pair_inv_scale, workspace))
     return AHV_EINVAL;
-  if (!aligned16(vol_src) || !aligned16(tgt_feat) || !aligned16(R) || !aligned16(W1) || !aligned16(W2) ||
-      !aligned16(h1_saved) || !aligned16(workspace))
-    return AHV_EINVAL;
+  if (!all_aligned16(vol_src, tgt_feat, R, W1, W2, h1_saved, workspace)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
   return launch_score_tc_train(vol_src, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, scores, h1_saved, pair_inv_scale, B, N,
@@ -164,10 +196,10 @@ AHV_API int ahv_score_backward_saved(const float* vol_src, const float* tgt_feat
                                      const float* grad_scores, const void* h1_saved, const float* pair_inv_scale,
                                      float* grad_vol, float* grad_tgt, float* grad_W1, float* grad_W2, float* grad_b2,
                                      int B, int64_t N, int math_mode, void* stream) {
-  if (B < 0 || N < 0 || N > 0x7fffffffLL) return AHV_EINVAL;
+  if (B < 0 || !n_ok(N)) return AHV_EINVAL;
   if (math_mode != AHV_MATH_TC && math_mode != AHV_MATH_FP32) return AHV_EINVAL;
-  if ((int64_t)B * N > 0 && (!vol_src || !tgt_feat || !R || !W1 || !W2 || !b2 || !base || !grad_scores || !h1_saved ||
-                             !pair_inv_scale || !grad_vol || !grad_tgt || !grad_W1 || !grad_W2 || !grad_b2))
+  if ((int64_t)B * N > 0 && !all_set(vol_src, tgt_feat, R, W1, W2, b2, base, grad_scores, h1_saved, pair_inv_scale,
+                                      grad_vol, grad_tgt, grad_W1, grad_W2, grad_b2))
     return AHV_EINVAL;
   if (!aligned16(h1_saved)) return AHV_EINVAL;
   int st = check_device();
@@ -187,17 +219,13 @@ AHV_API int ahv_forward_3d2d(const float* vol, const float* W1, const float* W2,
   return launch_forward_3d2d(vol, W1, W2, b2, feat, m, (cudaStream_t)stream);
 }
 
-// workspace = [scores B*N fp32 | top-k partial keys | tensor-core path scratch | per-shard top-k lists]
 AHV_API size_t ahv_workspace_bytes(int B, int64_t N, int k) {
-  if (B < 0 || N < 0) return 0;
-  return align_up((size_t)B * (size_t)N * sizeof(float), 256) +
-         align_up(topk_workspace_bytes(B, N, k), 256) + align_up(score_tc_workspace_bytes(B, N), 256) +
-         align_up((size_t)B * (size_t)(k > 0 ? k : 1) * (sizeof(float) + sizeof(int64_t)), 256);
+  return B < 0 || N < 0 ? 0 : VerifyWs(B, N, k).total;
 }
 
 AHV_API int ahv_topk(const float* scores, int B, int64_t N, int k, int64_t idx_offset, float* topk_val,
              int64_t* topk_idx, void* workspace, size_t workspace_bytes, void* stream) {
-  if (B < 0 || N < 0 || N > 0x7fffffffLL || k < 1 || k > kMaxK) return AHV_EINVAL;
+  if (B < 0 || !n_ok(N) || !k_ok(k)) return AHV_EINVAL;
   if (B > 0 && (!scores || !topk_val || !topk_idx || !workspace)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
@@ -207,7 +235,7 @@ AHV_API int ahv_topk(const float* scores, int B, int64_t N, int k, int64_t idx_o
 
 AHV_API int ahv_topk_merge(const float* vals, const int64_t* idx, int parts, int B, int k, float* out_val,
                    int64_t* out_idx, void* stream) {
-  if (parts < 1 || B < 0 || k < 1 || k > kMaxK) return AHV_EINVAL;
+  if (parts < 1 || B < 0 || !k_ok(k)) return AHV_EINVAL;
   if (B > 0 && (!vals || !idx || !out_val || !out_idx)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
@@ -228,30 +256,19 @@ AHV_API int ahv_score(const void* vol_src, int vol_dtype, const float* tgt_feat,
               int r_per_pair, const float* W1, const float* W2, const float* b2, const float* base,
               float* scores, float* topk_val, int64_t* topk_idx, int k, int64_t idx_offset, int B,
               int64_t N, int math_mode, void* workspace, size_t workspace_bytes, void* stream) {
-  if (B < 0 || N < 0 || N > 0x7fffffffLL) return AHV_EINVAL;
-  if (vol_dtype != AHV_VOL_F32 && vol_dtype != AHV_VOL_BF16) return AHV_EINVAL;
-  if (math_mode != AHV_MATH_TC && math_mode != AHV_MATH_FP32 && math_mode != AHV_MATH_TC_F16GATHER) return AHV_EINVAL;
-  if (k < 0 || k > kMaxK) return AHV_EINVAL;
+  if (B < 0 || !n_ok(N) || !vol_dtype_ok(vol_dtype) || !math_mode_ok(math_mode)) return AHV_EINVAL;
+  if (k != 0 && !k_ok(k)) return AHV_EINVAL;  // k = 0: scores only
   if (k > 0 && (!topk_val || !topk_idx)) return AHV_EINVAL;
-  if ((int64_t)B * N > 0 && (!vol_src || !tgt_feat || !R || !W1 || !W2 || !b2 || !base))
-    return AHV_EINVAL;
-  if (!aligned16(vol_src) || !aligned16(tgt_feat) || !aligned16(R) || !aligned16(W1) ||
-      !aligned16(W2) || !aligned16(workspace))
-    return AHV_EINVAL;
+  if ((int64_t)B * N > 0 && !all_set(vol_src, tgt_feat, R, W1, W2, b2, base)) return AHV_EINVAL;
+  if (!all_aligned16(vol_src, tgt_feat, R, W1, W2, workspace)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
   if ((int64_t)B * N == 0) return AHV_OK;
 
-  // fixed layout [scores | top-k partials | tensor-core scratch], shared with ahv_verify
-  const size_t need_scores = align_up((size_t)B * (size_t)N * sizeof(float), 256);
-  const size_t need_topk = align_up(topk_workspace_bytes(B, N, k > 0 ? k : 1), 256);
-  const size_t need_tc = align_up(score_tc_workspace_bytes(B, N), 256);
-  if (need_scores + need_topk + need_tc > 0 && !workspace) return AHV_EWORKSPACE;
-  if (workspace_bytes < need_scores + need_topk + need_tc) return AHV_EWORKSPACE;
+  const VerifyWs w(B, N, k);
+  if (!workspace || workspace_bytes < w.lists) return AHV_EWORKSPACE;
   unsigned char* ws = static_cast<unsigned char*>(workspace);
   float* sc = scores ? scores : reinterpret_cast<float*>(ws);
-  void* ws_topk = ws + need_scores;
-  void* ws_tc = ws + need_scores + need_topk;
 
   cudaStream_t s = (cudaStream_t)stream;
   if (math_mode == AHV_MATH_FP32)
@@ -259,9 +276,9 @@ AHV_API int ahv_score(const void* vol_src, int vol_dtype, const float* tgt_feat,
                            N, s);
   else
     st = launch_score_tc(vol_src, vol_dtype, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, sc, B, N,
-                         ws_tc, need_tc, s, math_mode == AHV_MATH_TC_F16GATHER);
+                         ws + w.tc, w.lists - w.tc, s, math_mode == AHV_MATH_TC_F16GATHER);
   if (st != AHV_OK) return st;
-  if (k > 0) st = launch_topk(sc, B, N, k, idx_offset, topk_val, topk_idx, ws_topk, need_topk, s);
+  if (k > 0) st = launch_topk(sc, B, N, k, idx_offset, topk_val, topk_idx, ws + w.topk, w.tc - w.topk, s);
   return st;
 }
 
@@ -269,28 +286,20 @@ AHV_API int ahv_verify(const void* vol_src, int vol_dtype, const float* vol_tgt,
                        const float* W1, const float* W2, const float* b2, const float* base, float* scores,
                        float* topk_val, int64_t* topk_idx, float* R_best, int k, int64_t idx_offset, int B,
                        int64_t N, int math_mode, void* workspace, size_t workspace_bytes, void* stream) {
-  if (B < 0 || N < 0 || N > 0x7fffffffLL || k < 1 || k > kMaxK) return AHV_EINVAL;
-  if (vol_dtype != AHV_VOL_F32 && vol_dtype != AHV_VOL_BF16) return AHV_EINVAL;
-  if (math_mode != AHV_MATH_TC && math_mode != AHV_MATH_FP32 && math_mode != AHV_MATH_TC_F16GATHER) return AHV_EINVAL;
-  if ((int64_t)B * N > 0 && (!vol_src || !vol_tgt || !R || !W1 || !W2 || !b2 || !base || !topk_val || !topk_idx))
-    return AHV_EINVAL;
-  if (!aligned16(vol_src) || !aligned16(vol_tgt) || !aligned16(R) || !aligned16(W1) || !aligned16(W2) ||
-      !aligned16(workspace))
-    return AHV_EINVAL;
+  if (B < 0 || !n_ok(N) || !k_ok(k) || !vol_dtype_ok(vol_dtype) || !math_mode_ok(math_mode)) return AHV_EINVAL;
+  if ((int64_t)B * N > 0 && !all_set(vol_src, vol_tgt, R, W1, W2, b2, base, topk_val, topk_idx)) return AHV_EINVAL;
+  if (!all_aligned16(vol_src, vol_tgt, R, W1, W2, workspace)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
   if ((int64_t)B * N == 0) return AHV_OK;
-  if (!workspace || workspace_bytes < ahv_workspace_bytes(B, N, k)) return AHV_EWORKSPACE;
+  const VerifyWs w(B, N, k);
+  if (!workspace || workspace_bytes < w.total) return AHV_EWORKSPACE;
   cudaStream_t s = (cudaStream_t)stream;
-  // workspace = [scores | top-k partials | tensor-core scratch (packed weights, target features, scales, keys)]
-  unsigned char* ws = static_cast<unsigned char*>(workspace);
-  const size_t off_topk = align_up((size_t)B * (size_t)N * sizeof(float), 256);
-  const size_t off_tc = off_topk + align_up(topk_workspace_bytes(B, N, k), 256);
-  void* ws_tc = ws + off_tc;
+  void* ws_tc = static_cast<unsigned char*>(workspace) + w.tc;  // packed weights, target features, scales, keys
   if (math_mode != AHV_MATH_FP32 && k == 1)  // three launches, nothing but 40 B per hypothesis touches HBM
     return launch_verify_tc_argmax(vol_src, vol_dtype, vol_tgt, R, r_per_pair != 0, W1, W2, b2, base, scores,
                                    topk_val, topk_idx, R_best, idx_offset, B, N, ws_tc,
-                                   workspace_bytes - off_tc, s, math_mode == AHV_MATH_TC_F16GATHER);
+                                   workspace_bytes - w.tc, s, math_mode == AHV_MATH_TC_F16GATHER);
   float* tgt = scratch_tgt_feat(ws_tc, B);
   st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
   if (st != AHV_OK) return st;
@@ -304,8 +313,7 @@ AHV_API int ahv_verify(const void* vol_src, int vol_dtype, const float* vol_tgt,
 
 // ---- two-pass selection: dense set -> top-k -> local refinement (BASELINE config 4; extension) -----------
 AHV_API size_t ahv_refine_workspace_bytes(int B, int64_t N, int k, int m) {
-  if (B < 0 || N < 0 || k < 1 || k > kMaxK || m < 1) return 0;
-  return ahv_workspace_bytes(B, N, k) + ahv_workspace_bytes(B, (int64_t)k * m, 1);
+  return B < 0 || N < 0 || !k_ok(k) || m < 1 ? 0 : RefineWs(B, N, k, m).total;
 }
 
 AHV_API int ahv_refine(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
@@ -313,28 +321,28 @@ AHV_API int ahv_refine(const void* vol_src, int vol_dtype, const float* vol_tgt,
                        float max_angle_deg, uint64_t seed, float* first_val, int64_t* first_idx, float* first_R,
                        float* cand, float* best_val, int64_t* best_idx, float* R_best, int B, int64_t N,
                        int math_mode, void* workspace, size_t workspace_bytes, void* stream) {
-  if (B < 1 || N < 1 || k < 1 || k > kMaxK || k > N || m < 1 || (int64_t)k * m > 0x7fffffffLL) return AHV_EINVAL;
-  if (!first_val || !first_idx || !first_R || !cand || !best_val || !best_idx || !workspace) return AHV_EINVAL;
+  if (B < 1 || N < 1 || !k_ok(k) || k > N || m < 1 || !n_ok((int64_t)k * m)) return AHV_EINVAL;
+  if (!all_set(first_val, first_idx, first_R, cand, best_val, best_idx, workspace)) return AHV_EINVAL;
   if (!aligned16(cand)) return AHV_EINVAL;
-  const size_t ws1 = ahv_workspace_bytes(B, N, k), ws2 = ahv_workspace_bytes(B, (int64_t)k * m, 1);
-  if (workspace_bytes < ws1 + ws2) return AHV_EWORKSPACE;
+  const RefineWs w(B, N, k, m);
+  if (workspace_bytes < w.total) return AHV_EWORKSPACE;
   unsigned char* ws = static_cast<unsigned char*>(workspace);
   // pass 1: the whole set, top-k and their rotations
   int st = ahv_verify(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, first_val, first_idx, first_R, k,
-                      0, B, N, math_mode, ws, ws1, stream);
+                      0, B, N, math_mode, ws, w.cand, stream);
   if (st != AHV_OK) return st;
   // candidates: m rotations within max_angle_deg of each of the B*k winners (index 0 = the winner itself)
   st = ahv_so3_perturb(first_R, (int64_t)B * k, m, max_angle_deg, seed, cand, stream);
   if (st != AHV_OK) return st;
   // pass 2: per-pair candidate sets [B, k*m], arg-max
   return ahv_verify(vol_src, vol_dtype, vol_tgt, cand, 1, W1, W2, b2, base, nullptr, best_val, best_idx, R_best, 1, 0, B,
-                    (int64_t)k * m, math_mode, ws + ws1, ws2, stream);
+                    (int64_t)k * m, math_mode, ws + w.cand, w.total - w.cand, stream);
 }
 
 // ---- gradient ascent of the fp32 score on SO(3), alone and after the grid pass (extension) ---------------
 namespace {
 bool ascent_args_ok(int vol_dtype, int steps, float step_deg) {
-  return (vol_dtype == AHV_VOL_F32 || vol_dtype == AHV_VOL_BF16) && steps >= 0 && steps <= 1000 &&
+  return vol_dtype_ok(vol_dtype) && steps >= 0 && steps <= 1000 &&
          std::isfinite(step_deg) && step_deg > 0.0f;   // the step cap bounds the runtime of one launch
 }
 }  // namespace
@@ -343,21 +351,16 @@ AHV_API int ahv_gradient_ascent(const void* vol_src, int vol_dtype, const float*
                                 const float* W1, const float* W2, const float* b2, const float* base, int steps,
                                 float step_deg, float* R_out, float* score_out, int B, int K, void* stream) {
   if (B < 1 || K < 1 || !ascent_args_ok(vol_dtype, steps, step_deg)) return AHV_EINVAL;
-  if (!vol_src || !tgt_feat || !R_init || !W1 || !W2 || !b2 || !base || !R_out || !score_out) return AHV_EINVAL;
-  if (!aligned16(vol_src) || !aligned16(tgt_feat) || !aligned16(R_init) || !aligned16(R_out) || !aligned16(W1) ||
-      !aligned16(W2))
-    return AHV_EINVAL;
+  if (!all_set(vol_src, tgt_feat, R_init, W1, W2, b2, base, R_out, score_out)) return AHV_EINVAL;
+  if (!all_aligned16(vol_src, tgt_feat, R_init, R_out, W1, W2)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
   return launch_gradient_ascent(vol_src, vol_dtype, tgt_feat, R_init, W1, W2, b2, base, steps, step_deg, R_out, score_out,
                                 B, K, (cudaStream_t)stream);
 }
 
-// workspace = [ahv_verify's for the grid pass | target features B*32*64 fp32 | top-k partials over [B,k]]
 AHV_API size_t ahv_refine_gradient_workspace_bytes(int B, int64_t N, int k) {
-  if (B < 0 || N < 0 || k < 1 || k > kMaxK) return 0;
-  return ahv_workspace_bytes(B, N, k) + align_up((size_t)B * kO * kP * sizeof(float), 256) +
-         align_up(topk_workspace_bytes(B, k, 1), 256);
+  return B < 0 || N < 0 || !k_ok(k) ? 0 : RefineGradientWs(B, N, k).total;
 }
 
 namespace {
@@ -369,28 +372,24 @@ int refine_gradient(const void* vol_src, int vol_dtype, const float* vol_tgt, co
                     float* first_val, int64_t* first_idx, float* first_R, float* R_all, float* score_all, float* best_val,
                     int64_t* best_idx, float* R_best, int B, int64_t N, int math_mode, void* workspace,
                     size_t workspace_bytes, void* stream) {
-  if (B < 1 || N < 1 || N > 0x7fffffffLL || k < 1 || k > kMaxK || k > N) return AHV_EINVAL;
-  if (!ascent_args_ok(vol_dtype, steps, step_deg) || !min_sep_ok(min_sep_deg)) return AHV_EINVAL;
-  if (math_mode != AHV_MATH_TC && math_mode != AHV_MATH_FP32 && math_mode != AHV_MATH_TC_F16GATHER) return AHV_EINVAL;
-  if (!vol_src || !vol_tgt || !R || !W1 || !W2 || !b2 || !base || !first_val || !first_idx || !first_R || !R_all ||
-      !score_all || !best_val || !best_idx || !workspace)
+  if (B < 1 || N < 1 || !n_ok(N) || !k_ok(k) || k > N) return AHV_EINVAL;
+  if (!ascent_args_ok(vol_dtype, steps, step_deg) || !min_sep_ok(min_sep_deg) || !math_mode_ok(math_mode)) return AHV_EINVAL;
+  if (!all_set(vol_src, vol_tgt, R, W1, W2, b2, base, first_val, first_idx, first_R, R_all, score_all, best_val, best_idx,
+               workspace))
     return AHV_EINVAL;
-  if (!aligned16(vol_src) || !aligned16(vol_tgt) || !aligned16(R) || !aligned16(W1) || !aligned16(W2) ||
-      !aligned16(first_R) || !aligned16(R_all) || !aligned16(R_best) || !aligned16(workspace))
-    return AHV_EINVAL;
-  const size_t ws1 = ahv_workspace_bytes(B, N, k), ws_tgt = align_up((size_t)B * kO * kP * sizeof(float), 256);
-  const size_t ws_top = align_up(topk_workspace_bytes(B, k, 1), 256);
-  if (workspace_bytes < ws1 + ws_tgt + ws_top) return AHV_EWORKSPACE;
+  if (!all_aligned16(vol_src, vol_tgt, R, W1, W2, first_R, R_all, R_best, workspace)) return AHV_EINVAL;
+  const RefineGradientWs w(B, N, k);
+  if (workspace_bytes < w.total) return AHV_EWORKSPACE;
   int st = check_device();
   if (st != AHV_OK) return st;
   cudaStream_t s = (cudaStream_t)stream;
   unsigned char* ws = static_cast<unsigned char*>(workspace);
-  float* tgt = reinterpret_cast<float*>(ws + ws1);
+  float* tgt = reinterpret_cast<float*>(ws + w.tgt);
   const bool distinct = min_sep_deg > 0.0f;
   if (!distinct) {
     // pass 1: the whole set, top-k and their rotations
     st = ahv_verify(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, first_val, first_idx, first_R, k,
-                    0, B, N, math_mode, ws, ws1, stream);
+                    0, B, N, math_mode, ws, w.tgt, stream);
     if (st != AHV_OK) return st;
   }
   // the ascent scores in fp32 against fp32 target features (bit-equal to ahv_forward_3d2d), whatever math_mode is
@@ -399,7 +398,7 @@ int refine_gradient(const void* vol_src, int vol_dtype, const float* vol_tgt, co
   if (distinct) {
     // pass 1: every score of the set (the fused k = 1 arg-max writes none), then the k distinct winners
     st = ahv_score(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, nullptr, nullptr, nullptr, 0, 0, B, N,
-                   math_mode, ws, ws1, stream);
+                   math_mode, ws, w.tgt, stream);
     if (st != AHV_OK) return st;
     st = launch_topk_distinct(reinterpret_cast<const float*>(ws), R, r_per_pair != 0, B, N, k, min_sep_deg, first_val,
                               first_idx, first_R, s);
@@ -410,7 +409,7 @@ int refine_gradient(const void* vol_src, int vol_dtype, const float* vol_tgt, co
                               distinct ? first_idx : nullptr);
   if (st != AHV_OK) return st;
   // per-pair arg-max over the k ascended candidates
-  st = launch_topk(score_all, B, k, 1, 0, best_val, best_idx, ws + ws1 + ws_tgt, ws_top, s);
+  st = launch_topk(score_all, B, k, 1, 0, best_val, best_idx, ws + w.top, w.total - w.top, s);
   if (st != AHV_OK || !R_best) return st;
   return launch_gather_rotations(R_all, 1, best_idx, 0, B, k, 1, R_best, s);
 }
@@ -440,10 +439,10 @@ AHV_API int ahv_refine_gradient_distinct(const void* vol_src, int vol_dtype, con
 // ---- top-k of distinct rotations: greedy geodesic non-maximum suppression on SO(3) (extension) ------------
 AHV_API int ahv_topk_distinct(const float* scores, const float* R, int r_per_pair, int B, int64_t N, int k,
                               float min_sep_deg, float* topk_val, int64_t* topk_idx, float* R_best, void* stream) {
-  if (B < 0 || N < 0 || N > 0x7fffffffLL || k < 1 || k > kMaxK || !min_sep_ok(min_sep_deg)) return AHV_EINVAL;
+  if (B < 0 || !n_ok(N) || !k_ok(k) || !min_sep_ok(min_sep_deg)) return AHV_EINVAL;
   if (B > 0 && (!topk_val || !topk_idx)) return AHV_EINVAL;
   if ((int64_t)B * N > 0 && (!scores || !R)) return AHV_EINVAL;
-  if (!aligned16(R) || !aligned16(R_best)) return AHV_EINVAL;
+  if (!all_aligned16(R, R_best)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
   return launch_topk_distinct(scores, R, r_per_pair != 0, B, N, k, min_sep_deg, topk_val, topk_idx, R_best,
@@ -452,11 +451,11 @@ AHV_API int ahv_topk_distinct(const float* scores, const float* R, int r_per_pai
 
 // ---- hypothesis set sharded over the GPUs of one node: winners exchanged through peer memory -------------
 AHV_API size_t ahv_peer_bytes(int max_pairs, int max_k) {
-  return (max_pairs < 1 || max_k < 1 || max_k > kMaxK) ? 0 : peer::buffer_bytes(max_pairs, max_k);
+  return (max_pairs < 1 || !k_ok(max_k)) ? 0 : peer::buffer_bytes(max_pairs, max_k);
 }
 
 AHV_API int ahv_peer_alloc(int max_pairs, int max_k, void** ptr) {
-  if (!ptr || max_pairs < 1 || max_k < 1 || max_k > kMaxK) return AHV_EINVAL;
+  if (!ptr || max_pairs < 1 || !k_ok(max_k)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
   const size_t bytes = peer::buffer_bytes(max_pairs, max_k);
@@ -518,7 +517,7 @@ int make_peer_args(int rank, int world, void* const* peers, int peer_max_pairs, 
   pa->cap_pairs = peer_max_pairs;
   pa->cap_k = peer_max_k;
   if (world > 1) {
-    if (!peers || peer_max_pairs < 1 || peer_max_k < 1 || peer_max_k > kMaxK) return AHV_EINVAL;
+    if (!peers || peer_max_pairs < 1 || !k_ok(peer_max_k)) return AHV_EINVAL;
     for (int r = 0; r < world; ++r) {
       if (!peers[r]) return AHV_EINVAL;
       pa->bufs[r] = static_cast<unsigned char*>(peers[r]);
@@ -531,7 +530,7 @@ int make_peer_args(int rank, int world, void* const* peers, int peer_max_pairs, 
 AHV_API int ahv_topk_exchange(const float* val, const int64_t* idx, const float* R, int r_per_pair, int64_t idx_offset,
                               int64_t N, int B, int k, float* out_val, int64_t* out_idx, float* R_best, int rank,
                               int world, void* const* peers, int peer_max_pairs, int peer_max_k, void* stream) {
-  if (B < 1 || k < 1 || k > kMaxK || N < 0 || idx_offset < 0 || !val || !idx || !out_val || !out_idx || (N > 0 && !R))
+  if (B < 1 || !k_ok(k) || N < 0 || idx_offset < 0 || !val || !idx || !out_val || !out_idx || (N > 0 && !R))
     return AHV_EINVAL;
   if (idx_offset + N > 0x100000000LL) return AHV_EINVAL;  // keys carry 32 index bits
   peer::Args pa;
@@ -549,14 +548,11 @@ AHV_API int ahv_verify_sharded(const void* vol_src, int vol_dtype, const float* 
                                int64_t* topk_idx, float* R_best, int k, int64_t idx_offset, int B, int64_t N,
                                int math_mode, void* workspace, size_t workspace_bytes, int rank, int world,
                                void* const* peers, int peer_max_pairs, int peer_max_k, void* stream) {
-  if (B < 1 || N < 0 || N > 0x7fffffffLL || k < 1 || k > kMaxK || idx_offset < 0) return AHV_EINVAL;
+  if (B < 1 || !n_ok(N) || !k_ok(k) || idx_offset < 0) return AHV_EINVAL;
   if (idx_offset + N > 0x100000000LL) return AHV_EINVAL;  // keys carry 32 index bits
-  if (vol_dtype != AHV_VOL_F32 && vol_dtype != AHV_VOL_BF16) return AHV_EINVAL;
-  if (math_mode != AHV_MATH_TC && math_mode != AHV_MATH_FP32 && math_mode != AHV_MATH_TC_F16GATHER) return AHV_EINVAL;
+  if (!vol_dtype_ok(vol_dtype) || !math_mode_ok(math_mode)) return AHV_EINVAL;
   if (!vol_src || !vol_tgt || (N > 0 && !R) || !W1 || !W2 || !b2 || !base || !topk_val || !topk_idx) return AHV_EINVAL;
-  if (!aligned16(vol_src) || !aligned16(vol_tgt) || !aligned16(R) || !aligned16(W1) || !aligned16(W2) ||
-      !aligned16(workspace))
-    return AHV_EINVAL;
+  if (!all_aligned16(vol_src, vol_tgt, R, W1, W2, workspace)) return AHV_EINVAL;
   peer::Args pa;
   int st = make_peer_args(rank, world, peers, peer_max_pairs, peer_max_k, &pa);
   if (st != AHV_OK) return st;
@@ -567,25 +563,24 @@ AHV_API int ahv_verify_sharded(const void* vol_src, int vol_dtype, const float* 
     return N == 0 ? AHV_EINVAL
                   : ahv_verify(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, topk_val, topk_idx,
                                R_best, k, idx_offset, B, N, math_mode, workspace, workspace_bytes, stream);
-  if (!workspace || workspace_bytes < ahv_workspace_bytes(B, N, k)) return AHV_EWORKSPACE;
+  const VerifyWs w(B, N, k);
+  if (!workspace || workspace_bytes < w.total) return AHV_EWORKSPACE;
   unsigned char* ws = static_cast<unsigned char*>(workspace);
-  const size_t off_tc = align_up((size_t)B * (size_t)N * sizeof(float), 256) + align_up(topk_workspace_bytes(B, N, k), 256);
-  const size_t need_tc = align_up(score_tc_workspace_bytes(B, N), 256);
   cudaStream_t s = (cudaStream_t)stream;
   if (k == 1 && N > 0 && math_mode != AHV_MATH_FP32)  // the scoring kernel exchanges and merges the winners itself
     return launch_verify_tc_argmax(vol_src, vol_dtype, vol_tgt, R, r_per_pair != 0, W1, W2, b2, base, nullptr, topk_val,
-                                   topk_idx, R_best, idx_offset, B, N, ws + off_tc, need_tc, s,
+                                   topk_idx, R_best, idx_offset, B, N, ws + w.tc, w.lists - w.tc, s,
                                    math_mode == AHV_MATH_TC_F16GATHER, &pa);
   // k > 1 (or an empty shard, or fp32 FFMA arithmetic): local top-k of the shard, then the exchange kernel
-  float* l_val = reinterpret_cast<float*>(ws + off_tc + need_tc);
-  int64_t* l_idx = reinterpret_cast<int64_t*>(ws + off_tc + need_tc + align_up((size_t)B * k * sizeof(float), 8));
+  float* l_val = reinterpret_cast<float*>(ws + w.lists);
+  int64_t* l_idx = reinterpret_cast<int64_t*>(ws + w.lists + align_up((size_t)B * k * sizeof(float), 8));
   const int kl = N < k ? (int)N : k;
   if (kl < k) {  // pad with (-inf, -1), which the merge ignores
     AHV_CUDA_OK(cudaMemsetAsync(l_val, 0xff, (size_t)B * k * sizeof(float), s));
     AHV_CUDA_OK(cudaMemsetAsync(l_idx, 0xff, (size_t)B * k * sizeof(int64_t), s));
   }
   if (N > 0) {
-    float* tgt = scratch_tgt_feat(ws + off_tc, B);
+    float* tgt = scratch_tgt_feat(ws + w.tc, B);
     st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
     if (st != AHV_OK) return st;
     if (kl == k) {
@@ -639,9 +634,9 @@ AHV_API int ahv_predict_host_ex(ahv_host_session* session, const void* vol_src_h
                                 float* topk_val_host, int64_t* topk_idx_host, float* R_best_host, int k,
                                 int64_t idx_offset, int B, int64_t N, int math_mode, int rank, int world,
                                 void* const* peers, int peer_max_pairs, int peer_max_k, void* stream) {
-  if (!session || B < 1 || N < 1 || k < 1 || k > kMaxK) return AHV_EINVAL;
-  if (vol_dtype != AHV_VOL_F32 && vol_dtype != AHV_VOL_BF16) return AHV_EINVAL;
-  if (!vol_src_host || !vol_tgt_host || !R_host || !W1_host || !W2_host || !b2_host || !base_host) return AHV_EINVAL;
+  if (!session || B < 1 || N < 1 || !k_ok(k)) return AHV_EINVAL;
+  if (!vol_dtype_ok(vol_dtype)) return AHV_EINVAL;
+  if (!all_set(vol_src_host, vol_tgt_host, R_host, W1_host, W2_host, b2_host, base_host)) return AHV_EINVAL;
   if (!topk_val_host || !topk_idx_host) return AHV_EINVAL;
   if (world > 1 && scores_host) return AHV_EINVAL;  // a sharded step returns the selection only
   int st = check_device();
@@ -654,7 +649,7 @@ AHV_API int ahv_predict_host_ex(ahv_host_session* session, const void* vol_src_h
   const size_t r_b = (size_t)(r_per_pair ? B : 1) * N * 9 * sizeof(float);
   const size_t w_b = (size_t)(kO * kK + kO * kO + kO + 8) * sizeof(float);
   const size_t out_b = (size_t)B * k * (sizeof(float) + sizeof(int64_t) + 9 * sizeof(float));
-  const size_t ws_b = ahv_workspace_bytes(B, N, k);
+  const size_t ws_b = VerifyWs(B, N, k).total;
   const size_t total = align_up(src_b, 256) + align_up(tgt_b, 256) + align_up(r_b, 256) + align_up(w_b, 256) +
                        align_up(out_b, 256) + ws_b;
   if (session->bytes < total) {  // grow (rare): the stream may still use the old block

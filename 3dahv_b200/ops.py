@@ -34,8 +34,10 @@ def base_coords(device=None) -> torch.Tensor:
     return _BASE_DEV[device]
 
 
-def _stream(t: torch.Tensor):
-    return torch.cuda.current_stream(t.device).cuda_stream
+def _call(name: str, device, *args) -> None:
+    """lib3dahv_b200's `name`(*args, current stream of `device`) with `device` current; raises on a failing status."""
+    with torch.cuda.device(device):
+        _lib.check(getattr(_lib.lib(), name)(*args, torch.cuda.current_stream(device).cuda_stream), name)
 
 
 def _dev(t: torch.Tensor, name: str, dtype=torch.float32) -> torch.Tensor:
@@ -49,32 +51,56 @@ def _dev(t: torch.Tensor, name: str, dtype=torch.float32) -> torch.Tensor:
     return t
 
 
+def _vol_src(vol_src):
+    """A bf16 source volume stays bf16, any other must be fp32: (tensor, AHV_VOL_* code)."""
+    if vol_src.dtype == torch.bfloat16:
+        return _dev(vol_src, "vol_src", torch.bfloat16), VOL_BF16
+    return _dev(vol_src, "vol_src"), VOL_F32
+
+
+def _head(W1, W2, b2):
+    """The verification head's weights as the kernels read them: W1 [32,384], W2 [32,32], b2 [32]."""
+    return _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+
+
+def _rotations(R, B: int):
+    """R [N,3,3] shared by the B pairs or [B,N,3,3] one set per pair -> (R, per_pair, N)."""
+    per_pair = R.dim() == 4
+    if per_pair and R.shape[0] != B:
+        raise ValueError("per-pair R must be [B,N,3,3]")
+    if tuple(R.shape[-2:]) != (3, 3):
+        raise ValueError("R must be [...,3,3]")
+    return R, per_pair, R.shape[1] if per_pair else R.shape[0]
+
+
+def _workspace(ws, need: int, device):
+    """`ws` if it holds `need` bytes, else a new buffer that does: (workspace, its size in bytes)."""
+    if ws is None or ws.numel() * ws.element_size() < need:
+        ws = torch.empty(max(need, 16), device=device, dtype=torch.uint8)
+    return ws, ws.numel() * ws.element_size()
+
+
 def rotations_from_normals(normals: torch.Tensor) -> torch.Tensor:
     """[n,4] normals (GPU) -> [n,3,3]; pytorch3d random_rotations arithmetic."""
     o = _dev(normals, "normals")
     n = o.shape[0]
     R = torch.empty(n, 3, 3, device=o.device, dtype=torch.float32)
-    with torch.cuda.device(o.device):
-        _lib.check(_lib.lib().ahv_so3_from_normals(o.data_ptr(), R.data_ptr(), n, _stream(o)), "ahv_so3_from_normals")
+    _call("ahv_so3_from_normals", o.device, o.data_ptr(), R.data_ptr(), n)
     return R
 
 
 def sample_rotations(n: int, seed: int, first_index: int = 0, device="cuda") -> torch.Tensor:
     """Native Philox sampler: hypothesis i depends only on (seed, first_index+i)."""
-    device = torch.device(device)
-    R = torch.empty(n, 3, 3, device=device, dtype=torch.float32)
-    with torch.cuda.device(device):
-        _lib.check(_lib.lib().ahv_so3_sample(seed & (2**64 - 1), first_index, R.data_ptr(), n, _stream(R)), "ahv_so3_sample")
+    R = torch.empty(n, 3, 3, device=torch.device(device), dtype=torch.float32)
+    _call("ahv_so3_sample", R.device, seed & (2**64 - 1), first_index, R.data_ptr(), n)
     return R
 
 
 def grid_rotations(n_total: int, first_index: int = 0, count: int | None = None, device="cuda") -> torch.Tensor:
     """Deterministic super-Fibonacci SO(3) grid, points [first, first+count) of n_total."""
-    device = torch.device(device)
     count = n_total - first_index if count is None else count
-    R = torch.empty(count, 3, 3, device=device, dtype=torch.float32)
-    with torch.cuda.device(device):
-        _lib.check(_lib.lib().ahv_so3_grid(n_total, first_index, R.data_ptr(), count, _stream(R)), "ahv_so3_grid")
+    R = torch.empty(count, 3, 3, device=torch.device(device), dtype=torch.float32)
+    _call("ahv_so3_grid", R.device, n_total, first_index, R.data_ptr(), count)
     return R
 
 
@@ -85,9 +111,7 @@ def perturb_rotations(R_center: torch.Tensor, m: int, max_angle_deg: float, seed
     lead = c.shape[:-2]
     n = c.numel() // 9
     out = torch.empty(*lead, m, 3, 3, device=c.device, dtype=torch.float32)
-    with torch.cuda.device(c.device):
-        _lib.check(_lib.lib().ahv_so3_perturb(c.data_ptr(), n, m, float(max_angle_deg), seed & (2**64 - 1), out.data_ptr(),
-                                              _stream(c)), "ahv_so3_perturb")
+    _call("ahv_so3_perturb", c.device, c.data_ptr(), n, m, float(max_angle_deg), seed & (2**64 - 1), out.data_ptr())
     return out
 
 
@@ -104,8 +128,7 @@ def rotate_volume(volume: torch.Tensor, R: torch.Tensor) -> torch.Tensor:
     v = _dev(volume, "volume")
     out = torch.empty(n, 16, 8, 8, 8, device=v.device, dtype=torch.float32)
     base = base_coords(v.device)
-    with torch.cuda.device(v.device):
-        _lib.check(_lib.lib().ahv_rotate_volume(v.data_ptr(), int(per_rot), R.data_ptr(), base.data_ptr(), out.data_ptr(), n, _stream(v)), "ahv_rotate_volume")
+    _call("ahv_rotate_volume", v.device, v.data_ptr(), int(per_rot), R.data_ptr(), base.data_ptr(), out.data_ptr(), n)
     return out
 
 
@@ -119,9 +142,8 @@ def rotate_volume_backward(grad_out: torch.Tensor, R: torch.Tensor, per_rotation
     out = (torch.empty(n, 16, 8, 8, 8, device=g.device, dtype=torch.float32) if per_rotation
            else torch.zeros(16, 8, 8, 8, device=g.device, dtype=torch.float32))
     base = base_coords(g.device)
-    with torch.cuda.device(g.device):
-        _lib.check(_lib.lib().ahv_rotate_volume_backward(g.data_ptr(), int(per_rotation), R.data_ptr(), base.data_ptr(),
-                                                         out.data_ptr(), n, _stream(g)), "ahv_rotate_volume_backward")
+    _call("ahv_rotate_volume_backward", g.device, g.data_ptr(), int(per_rotation), R.data_ptr(), base.data_ptr(), out.data_ptr(),
+          n)
     return out
 
 
@@ -136,9 +158,8 @@ def rotate_volume_grad_R(vol: torch.Tensor, grad_out: torch.Tensor, R: torch.Ten
         raise ValueError("vol must be [n,16,8,8,8] (per rotation) or [16,8,8,8] (shared)")
     out = torch.empty(n, 3, 3, device=g.device, dtype=torch.float32)
     base = base_coords(g.device)
-    with torch.cuda.device(g.device):
-        _lib.check(_lib.lib().ahv_rotate_volume_grad_R(v.data_ptr(), int(per_rotation), R.data_ptr(), base.data_ptr(), g.data_ptr(),
-                                                       out.data_ptr(), n, _stream(g)), "ahv_rotate_volume_grad_R")
+    _call("ahv_rotate_volume_grad_R", g.device, v.data_ptr(), int(per_rotation), R.data_ptr(), base.data_ptr(), g.data_ptr(),
+          out.data_ptr(), n)
     return out
 
 
@@ -148,49 +169,38 @@ def score_train(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tensor, 
     wants back: conv1's ReLU'd output of every item (fp16 [B*N,64,32], 4 KB per item) and per pair [B] the factor
     that turns it back into conv1's output (2^e1 / scale: the pair scale and W1's normaliser)."""
     vs, tf, R = _dev(vol_src, "vol_src"), _dev(tgt_feat, "tgt_feat"), _dev(R, "R")
-    W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+    W1, W2, b2 = _head(W1, W2, b2)
     B = vs.shape[0]
-    per_pair = R.dim() == 4
-    N = R.shape[1] if per_pair else R.shape[0]
-    if tuple(vs.shape) != (B, 16, 8, 8, 8) or tuple(tf.shape) != (B, 32, 64) or (per_pair and R.shape[0] != B):
+    if tuple(vs.shape) != (B, 16, 8, 8, 8) or tuple(tf.shape) != (B, 32, 64):
         raise ValueError("vol_src [B,16,8,8,8], tgt_feat [B,32,64], R [N,3,3] or [B,N,3,3] expected")
+    R, per_pair, N = _rotations(R, B)
     dev = vs.device
     scores = torch.empty(B, N, device=dev, dtype=torch.float32)
     h1 = torch.empty(B * N, 64, 32, device=dev, dtype=torch.float16)
     pair_inv = torch.empty(B, device=dev, dtype=torch.float32)
-    need = workspace_bytes(B, N, 1)
-    if workspace is None or workspace.numel() * workspace.element_size() < need:
-        workspace = torch.empty(max(need, 16), device=dev, dtype=torch.uint8)
-    base = base_coords(dev)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().ahv_score_train(vs.data_ptr(), tf.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(),
-                                              b2.data_ptr(), base.data_ptr(), scores.data_ptr(), h1.data_ptr(), pair_inv.data_ptr(),
-                                              B, N, workspace.data_ptr(), workspace.numel() * workspace.element_size(),
-                                              _stream(vs)), "ahv_score_train")
+    workspace, ws_bytes = _workspace(workspace, workspace_bytes(B, N, 1), dev)
+    _call("ahv_score_train", dev, vs.data_ptr(), tf.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(),
+          b2.data_ptr(), base_coords(dev).data_ptr(), scores.data_ptr(), h1.data_ptr(), pair_inv.data_ptr(), B, N,
+          workspace.data_ptr(), ws_bytes)
     return scores, h1, pair_inv
 
 
 def _score_backward_ex(vs, tg, R, W1, W2, b2, gs, h1, pi, outs, B, N, per_pair):
     """ahv_score_backward_ex into `outs` = (grad_vol, grad_tgt, grad_W1, grad_W2, grad_b2, grad_R), each a zeroed
     tensor or None."""
-    base = base_coords(vs.device)
     ptr = lambda t: t.data_ptr() if t is not None else None
-    with torch.cuda.device(vs.device):
-        _lib.check(_lib.lib().ahv_score_backward_ex(vs.data_ptr(), tg.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(),
-                                                    W2.data_ptr(), b2.data_ptr(), base.data_ptr(), gs.data_ptr(), ptr(h1), ptr(pi),
-                                                    *(ptr(t) for t in outs), B, N, _stream(vs)), "ahv_score_backward_ex")
+    _call("ahv_score_backward_ex", vs.device, vs.data_ptr(), tg.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(),
+          W2.data_ptr(), b2.data_ptr(), base_coords(vs.device).data_ptr(), gs.data_ptr(), ptr(h1), ptr(pi),
+          *(ptr(t) for t in outs), B, N)
 
 
 def _score_backward_args(vol_src, tgt_feat, R, W1, W2, b2, grad_scores):
     vs, tg, R, gs = _dev(vol_src, "vol_src"), _dev(tgt_feat, "tgt_feat"), _dev(R, "R"), _dev(grad_scores, "grad_scores")
-    W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+    W1, W2, b2 = _head(W1, W2, b2)
     B = vs.shape[0]
-    per_pair = R.dim() == 4
-    N = R.shape[1] if per_pair else R.shape[0]
+    R, per_pair, N = _rotations(R, B)
     if tuple(vs.shape) != (B, 16, 8, 8, 8) or tuple(tg.shape) != (B, 32, 64) or tuple(gs.shape) != (B, N):
         raise ValueError("vol_src [B,16,8,8,8], tgt_feat [B,32,64], grad_scores [B,N] expected")
-    if per_pair and R.shape[0] != B:
-        raise ValueError("per-pair rotations must be [B,N,3,3]")
     return vs, tg, R, W1, W2, b2, gs, B, N, per_pair
 
 
@@ -219,19 +229,13 @@ def score_backward(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tenso
         g_R = z(*R.shape)
         _score_backward_ex(vs, tg, R, W1, W2, b2, gs, h1, pi, (g_vol, g_tgt, g_w1, g_w2, g_b2, g_R), B, N, per_pair)
         return g_vol, g_tgt, g_w1, g_w2, g_b2, g_R
-    base = base_coords(dev)
-    with torch.cuda.device(dev):
-        if h1 is not None:
-            _lib.check(_lib.lib().ahv_score_backward_saved(vs.data_ptr(), tg.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(),
-                                                           W2.data_ptr(), b2.data_ptr(), base.data_ptr(), gs.data_ptr(),
-                                                           h1.data_ptr(), pi.data_ptr(), g_vol.data_ptr(), g_tgt.data_ptr(),
-                                                           g_w1.data_ptr(), g_w2.data_ptr(), g_b2.data_ptr(), B, N, int(math), _stream(vs)),
-                       "ahv_score_backward_saved")
-        else:
-            _lib.check(_lib.lib().ahv_score_backward(vs.data_ptr(), tg.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(),
-                                                     W2.data_ptr(), b2.data_ptr(), base.data_ptr(), gs.data_ptr(),
-                                                     g_vol.data_ptr(), g_tgt.data_ptr(), g_w1.data_ptr(), g_w2.data_ptr(),
-                                                     g_b2.data_ptr(), B, N, _stream(vs)), "ahv_score_backward")
+    head = (vs.data_ptr(), tg.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
+            base_coords(dev).data_ptr(), gs.data_ptr())
+    tail = (g_vol.data_ptr(), g_tgt.data_ptr(), g_w1.data_ptr(), g_w2.data_ptr(), g_b2.data_ptr(), B, N)
+    if h1 is not None:
+        _call("ahv_score_backward_saved", dev, *head, h1.data_ptr(), pi.data_ptr(), *tail, int(math))
+    else:
+        _call("ahv_score_backward", dev, *head, *tail)
     return g_vol, g_tgt, g_w1, g_w2, g_b2
 
 
@@ -256,10 +260,8 @@ def infonce(scores: torch.Tensor, sampled_R: torch.Tensor, gt_delta_R: torch.Ten
         raise ValueError("scores [B,N], sampled_R [N,3,3] or [B,N,3,3], gt_delta_R [B,3,3] expected")
     loss = torch.empty(B, device=s.device, dtype=torch.float32)
     grad = torch.empty(B, N, device=s.device, dtype=torch.float32) if want_grad else None
-    with torch.cuda.device(s.device):
-        _lib.check(_lib.lib().ahv_infonce(s.data_ptr(), R.data_ptr(), int(per_pair), g.data_ptr(), float(acc_thr_deg),
-                                          float(temperature), loss.data_ptr(), grad.data_ptr() if want_grad else None, B, N,
-                                          _stream(s)), "ahv_infonce")
+    _call("ahv_infonce", s.device, s.data_ptr(), R.data_ptr(), int(per_pair), g.data_ptr(), float(acc_thr_deg),
+          float(temperature), loss.data_ptr(), grad.data_ptr() if want_grad else None, B, N)
     return loss, grad
 
 
@@ -274,9 +276,7 @@ def resblock3d(x: torch.Tensor, conv1_w: torch.Tensor, conv2_w: torch.Tensor, do
         raise ValueError("weights must be conv1 [16,32,3,3,3], conv2 [16,16,3,3,3], downsample [16,32,1,1,1]")
     m = v.shape[0]
     out = torch.empty(m, 16, 8, 8, 8, device=v.device, dtype=torch.float32)
-    with torch.cuda.device(v.device):
-        _lib.check(_lib.lib().ahv_resblock3d(v.data_ptr(), w1.data_ptr(), w2.data_ptr(), wd.data_ptr(), out.data_ptr(), m,
-                                             _stream(v)), "ahv_resblock3d")
+    _call("ahv_resblock3d", v.device, v.data_ptr(), w1.data_ptr(), w2.data_ptr(), wd.data_ptr(), out.data_ptr(), m)
     return out
 
 
@@ -285,11 +285,10 @@ def forward_3d2d(vol: torch.Tensor, W1: torch.Tensor, W2: torch.Tensor, b2: torc
     v = _dev(vol, "vol")
     if tuple(v.shape[1:]) != (16, 8, 8, 8):
         raise ValueError("vol must be [m,16,8,8,8]")
-    W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+    W1, W2, b2 = _head(W1, W2, b2)
     m = v.shape[0]
     feat = torch.empty(m, 32, 64, device=v.device, dtype=torch.float32)
-    with torch.cuda.device(v.device):
-        _lib.check(_lib.lib().ahv_forward_3d2d(v.data_ptr(), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(), feat.data_ptr(), m, _stream(v)), "ahv_forward_3d2d")
+    _call("ahv_forward_3d2d", v.device, v.data_ptr(), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(), feat.data_ptr(), m)
     return feat
 
 
@@ -303,42 +302,27 @@ def score(vol_src, tgt_feat, R, W1, W2, b2, k: int = 1, idx_offset: int = 0, mat
 
     vol_src [B,16,8,8,8] fp32|bf16, tgt_feat [B,32,64], R [N,3,3] or [B,N,3,3].
     Returns (scores [B,N] or None, topk_val [B,k], topk_idx [B,k] int64)."""
-    if vol_src.dtype == torch.bfloat16:
-        vs, vdt = _dev(vol_src, "vol_src", torch.bfloat16), VOL_BF16
-    else:
-        vs, vdt = _dev(vol_src, "vol_src"), VOL_F32
+    vs, vdt = _vol_src(vol_src)
     B = vs.shape[0]
     if tuple(vs.shape[1:]) != (16, 8, 8, 8):
         raise ValueError("vol_src must be [B,16,8,8,8]")
     tf = _dev(tgt_feat, "tgt_feat")
     if tuple(tf.shape) != (B, 32, 64):
         raise ValueError("tgt_feat must be [B,32,64]")
-    R = _dev(R, "R")
-    per_pair = R.dim() == 4
-    if per_pair and R.shape[0] != B:
-        raise ValueError("per-pair R must be [B,N,3,3]")
-    if tuple(R.shape[-2:]) != (3, 3):
-        raise ValueError("R must be [...,3,3]")
-    N = R.shape[1] if per_pair else R.shape[0]
+    R, per_pair, N = _rotations(_dev(R, "R"), B)
     if k < 0 or k > 32:
         raise ValueError("k must be in [0,32]")
-    W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+    W1, W2, b2 = _head(W1, W2, b2)
     dev = vs.device
     scores = torch.empty(B, N, device=dev, dtype=torch.float32) if return_scores else None
     kk = max(k, 1)
     val = torch.empty(B, kk, device=dev, dtype=torch.float32)
     idx = torch.empty(B, kk, device=dev, dtype=torch.int64)
-    need = workspace_bytes(B, N, kk)
-    if workspace is None or workspace.numel() * workspace.element_size() < need:
-        workspace = torch.empty(max(need, 16), device=dev, dtype=torch.uint8)
-    base = base_coords(dev)
-    with torch.cuda.device(dev):
-        st = _lib.lib().ahv_score(
-            vs.data_ptr(), vdt, tf.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(),
-            b2.data_ptr(), base.data_ptr(), scores.data_ptr() if scores is not None else None,
-            val.data_ptr() if k > 0 else None, idx.data_ptr() if k > 0 else None, k, idx_offset, B, N,
-            math, workspace.data_ptr(), workspace.numel() * workspace.element_size(), _stream(vs))
-    _lib.check(st, "ahv_score")
+    workspace, ws_bytes = _workspace(workspace, workspace_bytes(B, N, kk), dev)
+    _call("ahv_score", dev, vs.data_ptr(), vdt, tf.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(),
+          b2.data_ptr(), base_coords(dev).data_ptr(), scores.data_ptr() if scores is not None else None,
+          val.data_ptr() if k > 0 else None, idx.data_ptr() if k > 0 else None, k, idx_offset, B, N, math,
+          workspace.data_ptr(), ws_bytes)
     if k == 0:
         return scores, None, None
     return scores, val, idx
@@ -348,40 +332,24 @@ def verify(vol_src, vol_tgt, R, W1, W2, b2, k: int = 1, idx_offset: int = 0, mat
            return_scores: bool = False, gather: bool = True, workspace: torch.Tensor | None = None):
     """ahv_verify: target features + fused scoring + selection + winner gather in one C call.
     Returns (scores|None, topk_val [B,k], topk_idx [B,k], R_best [B,k,3,3]|None)."""
-    if vol_src.dtype == torch.bfloat16:
-        vs, vdt = _dev(vol_src, "vol_src", torch.bfloat16), VOL_BF16
-    else:
-        vs, vdt = _dev(vol_src, "vol_src"), VOL_F32
+    vs, vdt = _vol_src(vol_src)
     vt = _dev(vol_tgt, "vol_tgt")
     B = vs.shape[0]
     if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
         raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
-    R = _dev(R, "R")
-    per_pair = R.dim() == 4
-    if per_pair and R.shape[0] != B:
-        raise ValueError("per-pair R must be [B,N,3,3]")
-    if tuple(R.shape[-2:]) != (3, 3):
-        raise ValueError("R must be [...,3,3]")
-    N = R.shape[1] if per_pair else R.shape[0]
+    R, per_pair, N = _rotations(_dev(R, "R"), B)
     if k < 1 or k > 32:
         raise ValueError("k must be in [1,32]")
-    W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+    W1, W2, b2 = _head(W1, W2, b2)
     dev = vs.device
     scores = torch.empty(B, N, device=dev, dtype=torch.float32) if return_scores else None
     val = torch.empty(B, k, device=dev, dtype=torch.float32)
     idx = torch.empty(B, k, device=dev, dtype=torch.int64)
     Rb = torch.empty(B, k, 3, 3, device=dev, dtype=torch.float32) if gather else None
-    need = workspace_bytes(B, N, k)
-    if workspace is None or workspace.numel() * workspace.element_size() < need:
-        workspace = torch.empty(max(need, 16), device=dev, dtype=torch.uint8)
-    base = base_coords(dev)
-    with torch.cuda.device(dev):
-        st = _lib.lib().ahv_verify(
-            vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
-            base.data_ptr(), scores.data_ptr() if scores is not None else None, val.data_ptr(), idx.data_ptr(),
-            Rb.data_ptr() if Rb is not None else None, k, idx_offset, B, N, math, workspace.data_ptr(),
-            workspace.numel() * workspace.element_size(), _stream(vs))
-    _lib.check(st, "ahv_verify")
+    workspace, ws_bytes = _workspace(workspace, workspace_bytes(B, N, k), dev)
+    _call("ahv_verify", dev, vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(),
+          b2.data_ptr(), base_coords(dev).data_ptr(), scores.data_ptr() if scores is not None else None, val.data_ptr(),
+          idx.data_ptr(), Rb.data_ptr() if Rb is not None else None, k, idx_offset, B, N, math, workspace.data_ptr(), ws_bytes)
     return scores, val, idx, Rb
 
 
@@ -391,19 +359,15 @@ def refine(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, m: int = 64, max_angle_
     torch ops, CUDA-graph capturable (pass `out` = the tuple a previous call returned to reuse its buffers).
     Returns (first_val [B,k], first_idx [B,k], first_R [B,k,3,3], cand [B,k*m,3,3], best_val [B], best_idx [B],
     R_best [B,3,3], workspace)."""
-    if vol_src.dtype == torch.bfloat16:
-        vs, vdt = _dev(vol_src, "vol_src", torch.bfloat16), VOL_BF16
-    else:
-        vs, vdt = _dev(vol_src, "vol_src"), VOL_F32
-    vt, R = _dev(vol_tgt, "vol_tgt"), _dev(R, "R")
+    vs, vdt = _vol_src(vol_src)
+    vt = _dev(vol_tgt, "vol_tgt")
     B = vs.shape[0]
-    per_pair = R.dim() == 4
-    N = R.shape[1] if per_pair else R.shape[0]
+    R, per_pair, N = _rotations(_dev(R, "R"), B)
     if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
         raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
     if not (1 <= k <= min(32, N)) or m < 1:
         raise ValueError("1 <= k <= min(32, N) and m >= 1 expected")
-    W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+    W1, W2, b2 = _head(W1, W2, b2)
     dev = vs.device
     if out is None:
         f = dict(device=dev, dtype=torch.float32)
@@ -411,23 +375,12 @@ def refine(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, m: int = 64, max_angle_
                torch.empty(B, k * m, 3, 3, **f), torch.empty(B, **f), torch.empty(B, device=dev, dtype=torch.int64),
                torch.empty(B, 3, 3, **f))
     fv, fi, fR, cand, bv, bi, bR = out[:7]
-    need = int(_lib.lib().ahv_refine_workspace_bytes(B, N, k, m))
-    if workspace is None or workspace.numel() * workspace.element_size() < need:
-        workspace = torch.empty(max(need, 16), device=dev, dtype=torch.uint8)
-    base = base_coords(dev)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().ahv_refine(
-            vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
-            base.data_ptr(), k, m, float(max_angle_deg), seed & (2**64 - 1), fv.data_ptr(), fi.data_ptr(), fR.data_ptr(),
-            cand.data_ptr(), bv.data_ptr(), bi.data_ptr(), bR.data_ptr(), B, N, math, workspace.data_ptr(),
-            workspace.numel() * workspace.element_size(), _stream(vs)), "ahv_refine")
+    workspace, ws_bytes = _workspace(workspace, int(_lib.lib().ahv_refine_workspace_bytes(B, N, k, m)), dev)
+    _call("ahv_refine", dev, vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(),
+          b2.data_ptr(), base_coords(dev).data_ptr(), k, m, float(max_angle_deg), seed & (2**64 - 1), fv.data_ptr(),
+          fi.data_ptr(), fR.data_ptr(), cand.data_ptr(), bv.data_ptr(), bi.data_ptr(), bR.data_ptr(), B, N, math,
+          workspace.data_ptr(), ws_bytes)
     return fv, fi, fR, cand, bv, bi, bR, workspace
-
-
-def _vol_src(vol_src):
-    if vol_src.dtype == torch.bfloat16:
-        return _dev(vol_src, "vol_src", torch.bfloat16), VOL_BF16
-    return _dev(vol_src, "vol_src"), VOL_F32
 
 
 def gradient_ascent(vol_src, tgt_feat, R_init, W1, W2, b2, steps: int = 20, step_deg: float = 1.0, out=None):
@@ -442,16 +395,13 @@ def gradient_ascent(vol_src, tgt_feat, R_init, W1, W2, b2, steps: int = 20, step
         raise ValueError("vol_src [B,16,8,8,8] and tgt_feat [B,32,64] expected")
     if R.dim() != 4 or R.shape[0] != B or tuple(R.shape[2:]) != (3, 3):
         raise ValueError("R_init must be [B,K,3,3]")
-    W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+    W1, W2, b2 = _head(W1, W2, b2)
     K = R.shape[1]
     if out is None:
         out = (torch.empty(B, K, 3, 3, device=vs.device, dtype=torch.float32), torch.empty(B, K, device=vs.device, dtype=torch.float32))
     R_out, s_out = out
-    base = base_coords(vs.device)
-    with torch.cuda.device(vs.device):
-        _lib.check(_lib.lib().ahv_gradient_ascent(vs.data_ptr(), vdt, tf.data_ptr(), R.data_ptr(), W1.data_ptr(), W2.data_ptr(),
-                                                  b2.data_ptr(), base.data_ptr(), int(steps), float(step_deg), R_out.data_ptr(),
-                                                  s_out.data_ptr(), B, K, _stream(vs)), "ahv_gradient_ascent")
+    _call("ahv_gradient_ascent", vs.device, vs.data_ptr(), vdt, tf.data_ptr(), R.data_ptr(), W1.data_ptr(), W2.data_ptr(),
+          b2.data_ptr(), base_coords(vs.device).data_ptr(), int(steps), float(step_deg), R_out.data_ptr(), s_out.data_ptr(), B, K)
     return R_out, s_out
 
 
@@ -464,15 +414,14 @@ def refine_gradient(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, steps: int = 2
     Returns (first_val [B,k], first_idx [B,k], first_R [B,k,3,3], R_all [B,k,3,3], score_all [B,k], best_val [B],
     best_idx [B], R_best [B,3,3], workspace)."""
     vs, vdt = _vol_src(vol_src)
-    vt, R = _dev(vol_tgt, "vol_tgt"), _dev(R, "R")
+    vt = _dev(vol_tgt, "vol_tgt")
     B = vs.shape[0]
-    per_pair = R.dim() == 4
-    N = R.shape[1] if per_pair else R.shape[0]
+    R, per_pair, N = _rotations(_dev(R, "R"), B)
     if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
         raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
     if not 1 <= k <= min(32, N):
         raise ValueError("1 <= k <= min(32, N) expected")
-    W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+    W1, W2, b2 = _head(W1, W2, b2)
     dev = vs.device
     if out is None:
         f = dict(device=dev, dtype=torch.float32)
@@ -480,19 +429,15 @@ def refine_gradient(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, steps: int = 2
                torch.empty(B, k, 3, 3, **f), torch.empty(B, k, **f), torch.empty(B, **f),
                torch.empty(B, device=dev, dtype=torch.int64), torch.empty(B, 3, 3, **f))
     fv, fi, fR, Ra, sa, bv, bi, bR = out[:8]
-    need = int(_lib.lib().ahv_refine_gradient_workspace_bytes(B, N, k))
-    if workspace is None or workspace.numel() * workspace.element_size() < need:
-        workspace = torch.empty(max(need, 16), device=dev, dtype=torch.uint8)
-    base = base_coords(dev)
+    workspace, ws_bytes = _workspace(workspace, int(_lib.lib().ahv_refine_gradient_workspace_bytes(B, N, k)), dev)
     head = (vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
-            base.data_ptr(), k, int(steps), float(step_deg))
+            base_coords(dev).data_ptr(), k, int(steps), float(step_deg))
     tail = (fv.data_ptr(), fi.data_ptr(), fR.data_ptr(), Ra.data_ptr(), sa.data_ptr(), bv.data_ptr(), bi.data_ptr(), bR.data_ptr(),
-            B, N, math, workspace.data_ptr(), workspace.numel() * workspace.element_size(), _stream(vs))
-    with torch.cuda.device(dev):
-        if min_sep_deg == 0:
-            _lib.check(_lib.lib().ahv_refine_gradient(*head, *tail), "ahv_refine_gradient")
-        else:
-            _lib.check(_lib.lib().ahv_refine_gradient_distinct(*head, float(min_sep_deg), *tail), "ahv_refine_gradient_distinct")
+            B, N, math, workspace.data_ptr(), ws_bytes)
+    if min_sep_deg == 0:
+        _call("ahv_refine_gradient", dev, *head, *tail)
+    else:
+        _call("ahv_refine_gradient_distinct", dev, *head, float(min_sep_deg), *tail)
     return fv, fi, fR, Ra, sa, bv, bi, bR, workspace
 
 
@@ -509,12 +454,12 @@ def verify_sharded(vol_src, vol_tgt, R, W1, W2, b2, idx_offset: int, peer, k: in
     them (k == 1 with tensor-core arithmetic: inside the scoring kernel; otherwise one exchange kernel after the
     shard's top-k).  Returns (topk_val [B,k], topk_idx [B,k] global, R_best [B,k,3,3]) over the whole set,
     identical on every rank.  An empty slice ([0,3,3]) is allowed."""
-    vs = _dev(vol_src, "vol_src", vol_src.dtype if vol_src.dtype == torch.bfloat16 else torch.float32)
-    vt, R = _dev(vol_tgt, "vol_tgt"), _dev(R, "R")
-    W1, W2, b2 = _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
+    vs, vdt = _vol_src(vol_src)
+    vt = _dev(vol_tgt, "vol_tgt")
+    R = _dev(R, "R")
+    W1, W2, b2 = _head(W1, W2, b2)
     B = vs.shape[0]
-    per_pair = R.dim() == 4
-    N = R.shape[1] if per_pair else R.shape[0]
+    R, per_pair, N = _rotations(R, B)
     if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
         raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
     if B > peer.max_pairs or k > peer.max_k:
@@ -523,16 +468,10 @@ def verify_sharded(vol_src, vol_tgt, R, W1, W2, b2, idx_offset: int, peer, k: in
     val = torch.empty(B, k, device=dev, dtype=torch.float32)
     idx = torch.empty(B, k, device=dev, dtype=torch.int64)
     Rb = torch.empty(B, k, 3, 3, device=dev, dtype=torch.float32)
-    need = workspace_bytes(B, N, k)
-    if workspace is None or workspace.numel() * workspace.element_size() < need:
-        workspace = torch.empty(max(need, 16), device=dev, dtype=torch.uint8)
-    base = base_coords(dev)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().ahv_verify_sharded(
-            vs.data_ptr(), VOL_BF16 if vs.dtype == torch.bfloat16 else VOL_F32, vt.data_ptr(), R.data_ptr() if N else None,
-            int(per_pair), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(), base.data_ptr(), val.data_ptr(), idx.data_ptr(),
-            Rb.data_ptr(), k, idx_offset, B, N, math, workspace.data_ptr(), workspace.numel() * workspace.element_size(),
-            peer.rank, peer.world, _peer_array(peer), peer.max_pairs, peer.max_k, _stream(vs)), "ahv_verify_sharded")
+    workspace, ws_bytes = _workspace(workspace, workspace_bytes(B, N, k), dev)
+    _call("ahv_verify_sharded", dev, vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr() if N else None, int(per_pair), W1.data_ptr(),
+          W2.data_ptr(), b2.data_ptr(), base_coords(dev).data_ptr(), val.data_ptr(), idx.data_ptr(), Rb.data_ptr(), k, idx_offset,
+          B, N, math, workspace.data_ptr(), ws_bytes, peer.rank, peer.world, _peer_array(peer), peer.max_pairs, peer.max_k)
     return val, idx, Rb
 
 
@@ -541,16 +480,13 @@ def topk_exchange(val, idx, R, idx_offset: int, peer):
     rank, with the winning rotations.  Returns (topk_val [B,k], topk_idx [B,k], R_best [B,k,3,3])."""
     v, i, R = _dev(val, "val"), _dev(idx, "idx", torch.int64), _dev(R, "R")
     B, k = v.shape
-    per_pair = R.dim() == 4
-    N = R.shape[1] if per_pair else R.shape[0]
+    R, per_pair, N = _rotations(R, B)
     dev = v.device
     out_v = torch.empty(B, k, device=dev, dtype=torch.float32)
     out_i = torch.empty(B, k, device=dev, dtype=torch.int64)
     Rb = torch.empty(B, k, 3, 3, device=dev, dtype=torch.float32)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().ahv_topk_exchange(v.data_ptr(), i.data_ptr(), R.data_ptr() if N else None, int(per_pair), idx_offset,
-                                                N, B, k, out_v.data_ptr(), out_i.data_ptr(), Rb.data_ptr(), peer.rank, peer.world,
-                                                _peer_array(peer), peer.max_pairs, peer.max_k, _stream(v)), "ahv_topk_exchange")
+    _call("ahv_topk_exchange", dev, v.data_ptr(), i.data_ptr(), R.data_ptr() if N else None, int(per_pair), idx_offset, N, B, k,
+          out_v.data_ptr(), out_i.data_ptr(), Rb.data_ptr(), peer.rank, peer.world, _peer_array(peer), peer.max_pairs, peer.max_k)
     return out_v, out_i, Rb
 
 
@@ -560,11 +496,8 @@ def topk(scores: torch.Tensor, k: int, idx_offset: int = 0):
     B, N = s.shape
     val = torch.empty(B, k, device=s.device, dtype=torch.float32)
     idx = torch.empty(B, k, device=s.device, dtype=torch.int64)
-    need = workspace_bytes(B, N, k)
-    ws = torch.empty(max(need, 16), device=s.device, dtype=torch.uint8)
-    with torch.cuda.device(s.device):
-        st = _lib.lib().ahv_topk(s.data_ptr(), B, N, k, idx_offset, val.data_ptr(), idx.data_ptr(), ws.data_ptr(), ws.numel(), _stream(s))
-    _lib.check(st, "ahv_topk")
+    ws, ws_bytes = _workspace(None, workspace_bytes(B, N, k), s.device)
+    _call("ahv_topk", s.device, s.data_ptr(), B, N, k, idx_offset, val.data_ptr(), idx.data_ptr(), ws.data_ptr(), ws_bytes)
     return val, idx
 
 
@@ -583,10 +516,8 @@ def topk_distinct(scores: torch.Tensor, R: torch.Tensor, k: int, min_sep_deg: fl
     val = torch.empty(B, k, device=s.device, dtype=torch.float32)
     idx = torch.empty(B, k, device=s.device, dtype=torch.int64)
     Rb = torch.empty(B, k, 3, 3, device=s.device, dtype=torch.float32) if gather else None
-    with torch.cuda.device(s.device):
-        st = _lib.lib().ahv_topk_distinct(s.data_ptr(), R.data_ptr(), int(per_pair), B, N, k, float(min_sep_deg), val.data_ptr(),
-                                          idx.data_ptr(), Rb.data_ptr() if gather else None, _stream(s))
-    _lib.check(st, "ahv_topk_distinct")
+    _call("ahv_topk_distinct", s.device, s.data_ptr(), R.data_ptr(), int(per_pair), B, N, k, float(min_sep_deg), val.data_ptr(),
+          idx.data_ptr(), Rb.data_ptr() if gather else None)
     return val, idx, Rb
 
 
@@ -596,22 +527,17 @@ def topk_merge(vals: torch.Tensor, idx: torch.Tensor):
     parts, B, k = v.shape
     out_v = torch.empty(B, k, device=v.device, dtype=torch.float32)
     out_i = torch.empty(B, k, device=v.device, dtype=torch.int64)
-    with torch.cuda.device(v.device):
-        st = _lib.lib().ahv_topk_merge(v.data_ptr(), i.data_ptr(), parts, B, k, out_v.data_ptr(), out_i.data_ptr(), _stream(v))
-    _lib.check(st, "ahv_topk_merge")
+    _call("ahv_topk_merge", v.device, v.data_ptr(), i.data_ptr(), parts, B, k, out_v.data_ptr(), out_i.data_ptr())
     return out_v, out_i
 
 
 def gather_rotations(R: torch.Tensor, idx: torch.Tensor, idx_offset: int = 0) -> torch.Tensor:
     """sampled_R[pred_index] (modules/model.py:196): [B,k,3,3]."""
     R, idx = _dev(R, "R"), _dev(idx, "idx", torch.int64)
-    per_pair = R.dim() == 4
     B, k = idx.shape
-    N = R.shape[1] if per_pair else R.shape[0]
+    R, per_pair, N = _rotations(R, B)
     out = torch.empty(B, k, 3, 3, device=R.device, dtype=torch.float32)
-    with torch.cuda.device(R.device):
-        st = _lib.lib().ahv_gather_rotations(R.data_ptr(), int(per_pair), idx.data_ptr(), idx_offset, B, N, k, out.data_ptr(), _stream(R))
-    _lib.check(st, "ahv_gather_rotations")
+    _call("ahv_gather_rotations", R.device, R.data_ptr(), int(per_pair), idx.data_ptr(), idx_offset, B, N, k, out.data_ptr())
     return out
 
 
@@ -648,36 +574,29 @@ def predict_host(vol_src, vol_tgt, R, W1, W2, b2, k: int = 1, math: int = MATH_T
     if vs.is_cuda or vt.is_cuda or Rc.is_cuda:
         raise RuntimeError("predict_host takes host tensors")
     W1c, W2c, b2c = W1.reshape(32, 384).to(f).contiguous().cpu(), W2.reshape(32, 32).to(f).contiguous().cpu(), b2.to(f).contiguous().cpu()
-    per_pair = Rc.dim() == 4
     B = vs.shape[0]
-    N = Rc.shape[1] if per_pair else Rc.shape[0]
+    Rc, per_pair, N = _rotations(Rc, B)
     scores = torch.empty(B, N, dtype=f) if return_scores else None
     val = torch.empty(B, k, dtype=f)
     idx = torch.empty(B, k, dtype=torch.int64)
     Rb = torch.empty(B, k, 3, 3, dtype=f)
     base = base_coords()
     device = torch.device(device)
+    sc = scores.data_ptr() if scores is not None else None
     extended = session is not None or bf16 or idx_offset != 0 or peer is not None
-    with torch.cuda.device(device):
-        stream = torch.cuda.current_stream(device).cuda_stream
-        if not extended:
-            st = _lib.lib().ahv_predict_host(
-                vs.data_ptr(), vt.data_ptr(), Rc.data_ptr(), int(per_pair), W1c.data_ptr(), W2c.data_ptr(), b2c.data_ptr(),
-                base.data_ptr(), scores.data_ptr() if scores is not None else None, val.data_ptr(), idx.data_ptr(),
-                Rb.data_ptr(), k, B, N, math, stream)
-        else:
-            own = session is None
-            if own:
-                session = HostSession(device)
-            try:
-                st = _lib.lib().ahv_predict_host_ex(
-                    session.handle, vs.data_ptr(), VOL_BF16 if bf16 else VOL_F32, vt.data_ptr(), Rc.data_ptr(), int(per_pair),
-                    W1c.data_ptr(), W2c.data_ptr(), b2c.data_ptr(), base.data_ptr(),
-                    scores.data_ptr() if scores is not None else None, val.data_ptr(), idx.data_ptr(), Rb.data_ptr(), k,
-                    idx_offset, B, N, math, peer.rank if peer else 0, peer.world if peer else 1,
-                    _peer_array(peer) if peer else None, peer.max_pairs if peer else 0, peer.max_k if peer else 0, stream)
-            finally:
-                if own:
-                    session.close()
-    _lib.check(st, "ahv_predict_host")
+    if not extended:
+        _call("ahv_predict_host", device, vs.data_ptr(), vt.data_ptr(), Rc.data_ptr(), int(per_pair), W1c.data_ptr(),
+              W2c.data_ptr(), b2c.data_ptr(), base.data_ptr(), sc, val.data_ptr(), idx.data_ptr(), Rb.data_ptr(), k, B, N, math)
+        return scores, val, idx, Rb
+    own = session is None
+    if own:
+        session = HostSession(device)
+    try:
+        _call("ahv_predict_host_ex", device, session.handle, vs.data_ptr(), VOL_BF16 if bf16 else VOL_F32, vt.data_ptr(),
+              Rc.data_ptr(), int(per_pair), W1c.data_ptr(), W2c.data_ptr(), b2c.data_ptr(), base.data_ptr(), sc, val.data_ptr(),
+              idx.data_ptr(), Rb.data_ptr(), k, idx_offset, B, N, math, peer.rank if peer else 0, peer.world if peer else 1,
+              _peer_array(peer) if peer else None, peer.max_pairs if peer else 0, peer.max_k if peer else 0)
+    finally:
+        if own:
+            session.close()
     return scores, val, idx, Rb

@@ -22,6 +22,17 @@ from ._lib import MATH_FP32, MATH_TC, MATH_TC_F16GATHER
 DEFAULT_MATH = MATH_TC
 
 
+def _src_volume(vol_src):
+    """A bf16 source volume as it is, any other as fp32: the two dtypes the scoring kernels read."""
+    return vol_src if vol_src.dtype == torch.bfloat16 else vol_src.float()
+
+
+def _clamp_k(k: int, R):
+    """(min(k, N), N) for a rotation set R [N,3,3] (shared) or [B,N,3,3] (per pair)."""
+    N = R.shape[1] if R.dim() == 4 else R.shape[0]
+    return min(k, N), N
+
+
 @dataclass
 class VerifyResult:
     scores: torch.Tensor | None    # [B,N] pred_sim (modules/model.py:193)
@@ -73,14 +84,11 @@ class HypothesisVerifier:
         rotations that lie pairwise more than min_sep_deg apart (`ops.topk_distinct`; empty slots are -inf / -1 / NaN)."""
         dev = vol_src.device
         W1, W2, b2 = self._weights_on(dev)
-        per_pair = R.dim() == 4
-        N = R.shape[1] if per_pair else R.shape[0]
-        B = vol_src.shape[0]
+        k, N = _clamp_k(k, R)
         if N == 0:
             raise ValueError("empty hypothesis set")
-        k = min(k, N)
-        vs = vol_src if vol_src.dtype == torch.bfloat16 else vol_src.float()
-        ws = self._workspace(B, N, k, dev)
+        vs = _src_volume(vol_src)
+        ws = self._workspace(vol_src.shape[0], N, k, dev)
         if min_sep_deg > 0:   # greedy NMS does not compose from per-shard lists: no idx_offset
             if idx_offset:
                 raise ValueError("min_sep_deg > 0 selects over the whole set: idx_offset must be 0")
@@ -109,14 +117,11 @@ class HypothesisVerifier:
         """Two-pass selection (BASELINE config 4; extension): score the set, keep the top-k, score m local
         perturbations of each, return the best - one C call (`ahv_refine`), no torch ops in between.
         Returns (R_best [B,3,3], score [B], first pass as a VerifyResult, candidate set [B,k*m,3,3])."""
-        dev = vol_src.device
-        W1, W2, b2 = self._weights_on(dev)
-        per_pair = R.dim() == 4
-        k = min(k, R.shape[1] if per_pair else R.shape[0])
-        vs = vol_src if vol_src.dtype == torch.bfloat16 else vol_src.float()
-        fv, fi, fR, cand, bv, bi, bR, self._ws_refine = ops.refine(vs, vol_tgt.float(), R, W1, W2, b2, k=k, m=m,
-                                                                  max_angle_deg=max_angle_deg, seed=seed, math=self.math,
-                                                                  workspace=getattr(self, "_ws_refine", None))
+        W1, W2, b2 = self._weights_on(vol_src.device)
+        k, _ = _clamp_k(k, R)
+        fv, fi, fR, cand, bv, bi, bR, self._ws_refine = ops.refine(
+            _src_volume(vol_src), vol_tgt.float(), R, W1, W2, b2, k=k, m=m, max_angle_deg=max_angle_deg, seed=seed,
+            math=self.math, workspace=getattr(self, "_ws_refine", None))
         return bR, bv, VerifyResult(None, fv, fi, fR), cand
 
     @torch.no_grad()
@@ -171,8 +176,8 @@ class HypothesisVerifier:
         score [B], R_all [B,k,3,3], score_all [B,k]); the best is the per-pair arg-max over k, ties to the lowest index."""
         W1, W2, b2 = self._weights_on(vol_src.device)
         R = (R_init[:, None] if R_init.dim() == 3 else R_init).float()
-        vs = vol_src if vol_src.dtype == torch.bfloat16 else vol_src.float()
-        R_all, s_all = ops.gradient_ascent(vs, self.target_features(vol_tgt), R, W1, W2, b2, steps=steps, step_deg=step_deg)
+        R_all, s_all = ops.gradient_ascent(_src_volume(vol_src), self.target_features(vol_tgt), R, W1, W2, b2, steps=steps,
+                                           step_deg=step_deg)
         val, idx = ops.topk(s_all, 1)
         return ops.gather_rotations(R_all, idx)[:, 0], val[:, 0], R_all, s_all
 
@@ -185,12 +190,19 @@ class HypothesisVerifier:
         (`ahv_refine_gradient_distinct`), so the ascents start in distinct basins; slots left empty are not ascended.
         Returns (R_best [B,3,3], score [B], first pass as a VerifyResult, R_all [B,k,3,3], score_all [B,k])."""
         W1, W2, b2 = self._weights_on(vol_src.device)
-        k = min(k, R.shape[1] if R.dim() == 4 else R.shape[0])
-        vs = vol_src if vol_src.dtype == torch.bfloat16 else vol_src.float()
+        k, _ = _clamp_k(k, R)
         fv, fi, fR, Ra, sa, bv, bi, bR, self._ws_refine_gradient = ops.refine_gradient(
-            vs, vol_tgt.float(), R, W1, W2, b2, k=k, steps=steps, step_deg=step_deg, math=self.math,
+            _src_volume(vol_src), vol_tgt.float(), R, W1, W2, b2, k=k, steps=steps, step_deg=step_deg, math=self.math,
             workspace=getattr(self, "_ws_refine_gradient", None), min_sep_deg=min_sep_deg)
         return bR, bv, VerifyResult(None, fv, fi, fR), Ra, sa
+
+
+def _replay(graph, *inputs):
+    """Copies each given (static buffer, new value) pair's value into its buffer, then replays `graph`."""
+    for buf, x in inputs:
+        if x is not None:
+            buf.copy_(x, non_blocking=True)
+    graph.replay()
 
 
 def _hat(u: torch.Tensor) -> torch.Tensor:
@@ -242,13 +254,7 @@ class GraphedVerifier:
 
     @torch.no_grad()
     def __call__(self, vol_src=None, vol_tgt=None, R=None) -> VerifyResult:
-        if vol_src is not None:
-            self.vol_src.copy_(vol_src, non_blocking=True)
-        if vol_tgt is not None:
-            self.vol_tgt.copy_(vol_tgt, non_blocking=True)
-        if R is not None:
-            self.R.copy_(R, non_blocking=True)
-        self.graph.replay()
+        _replay(self.graph, (self.vol_src, vol_src), (self.vol_tgt, vol_tgt), (self.R, R))
         return self.out
 
     def check(self) -> int:
@@ -309,13 +315,7 @@ class GraphedRefiner:
     def __call__(self, vol_src=None, vol_tgt=None, R=None):
         """Returns (R_best [B,3,3], score [B]); `.first` holds the first pass's top-k, `.candidates` the refinement set
         (method="perturb") or `.R_all` / `.score_all` the ascended top-k (method="gradient")."""
-        if vol_src is not None:
-            self.vol_src.copy_(vol_src, non_blocking=True)
-        if vol_tgt is not None:
-            self.vol_tgt.copy_(vol_tgt, non_blocking=True)
-        if R is not None:
-            self.R.copy_(R, non_blocking=True)
-        self.graph.replay()
+        _replay(self.graph, (self.vol_src, vol_src), (self.vol_tgt, vol_tgt), (self.R, R))
         return self.R_best, self.best_val
 
 
@@ -354,11 +354,5 @@ class GraphedTail:
 
     @torch.no_grad()
     def __call__(self, feat_src=None, feat_tgt=None, R=None) -> VerifyResult:
-        if feat_src is not None:
-            self.feat_src.copy_(feat_src, non_blocking=True)
-        if feat_tgt is not None:
-            self.feat_tgt.copy_(feat_tgt, non_blocking=True)
-        if R is not None:
-            self.R.copy_(R, non_blocking=True)
-        self.graph.replay()
+        _replay(self.graph, (self.feat_src, feat_src), (self.feat_tgt, feat_tgt), (self.R, R))
         return self.out
