@@ -252,7 +252,11 @@ def score_grad_R(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tensor,
 
 def infonce(scores: torch.Tensor, sampled_R: torch.Tensor, gt_delta_R: torch.Tensor, acc_thr_deg: float,
             temperature: float = 0.1, want_grad: bool = True):
-    """ahv_infonce: (loss [B], d loss / d scores [B,N] or None) in one launch (modules/model.py:43-63)."""
+    """ahv_infonce: (loss [B], d loss / d scores [B,N] or None) in one launch (modules/model.py:43-63).
+    The masses of the positives and the negatives are summed apart in double, so confident pairs (loss far below
+    fp32's epsilon) keep fp32 relative accuracy in the loss and in every gradient.  Domain: exp(scores/T) is fp32,
+    so |scores|/T must stay below ~88; the reference overflows there too.  Scores that are means of cosines lie in
+    [-1, 1] and cannot reach it at T = 0.1."""
     s, R, g = _dev(scores, "scores"), _dev(sampled_R, "sampled_R"), _dev(gt_delta_R, "gt_delta_R")
     B, N = s.shape
     per_pair = R.dim() == 4

@@ -51,9 +51,12 @@ class ResNetBlock_3D(_ResNetBlock):
     def forward(self, x):
         """modules/modules.py:32-47.  Inference on the GPU at the model's shape (32 -> 16 on 8^3, :100-101): one
         cluster launch (`ahv_resblock3d`, the step right before the hypothesis-and-verification path);
-        otherwise - training, CPU, other shapes - the PyTorch convolutions."""
+        otherwise - training, CPU, other shapes - the PyTorch convolutions.  The kernel has no backward, so it runs only
+        when nothing the block computes can need a gradient: grad mode off, or neither x nor any weight forward reads
+        (conv1, conv2, downsample) requires one.  `bn_down` never enters forward."""
+        weights = (self.conv1.weight, self.conv2.weight, self.downsample[0].weight) if self._fusable else ()
         if (self._fusable and x.is_cuda and x.dtype == torch.float32 and tuple(x.shape[1:]) == (32, 8, 8, 8)
-                and not (torch.is_grad_enabled() and (x.requires_grad or self.conv1.weight.requires_grad))):
+                and not (torch.is_grad_enabled() and (x.requires_grad or any(w.requires_grad for w in weights)))):
             return _ahv().ops.resblock3d(x, self.conv1.weight.detach(), self.conv2.weight.detach(),
                                          self.downsample[0].weight.detach())
         return super().forward(x)

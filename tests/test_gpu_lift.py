@@ -13,9 +13,11 @@ def test_resblock3d_vs_reference_fixture(ahv, golden_lift, oracle):
     T = lambda a: torch.from_numpy(a).to(DEV)
     out = ahv.ops.resblock3d(T(g["x"]), T(g["conv1_w"]), T(g["conv2_w"]), T(g["down_w"])).cpu().numpy()
     np.testing.assert_allclose(out, g["out"], atol=3e-6, rtol=0)          # the reference's own module, fp32 CPU
-    # ragged batch sizes against the restatement (clusters of 8 CTAs per volume; 1, 2 and 19 volumes)
+    # ragged batch sizes against the restatement (clusters of 8 CTAs per volume, one CTA per SM: 1, 2 and one more
+    # volume than there are resident clusters)
     gen = torch.Generator().manual_seed(1)
-    for m in (1, 2, 19):
+    resident = max(torch.cuda.get_device_properties(DEV).multi_processor_count // 8, 1)
+    for m in (1, 2, resident + 1):
         x = torch.randn(m, 32, 8, 8, 8, generator=gen)
         want = oracle.resblock3d_np(x.numpy(), g["conv1_w"], g["conv2_w"], g["down_w"])
         got = ahv.ops.resblock3d(x.to(DEV), T(g["conv1_w"]), T(g["conv2_w"]), T(g["down_w"])).cpu().numpy()
