@@ -159,6 +159,33 @@ AHV_API int ahv_score_backward_ex(const float* vol_src, const float* tgt_feat, c
                           grad_W1, grad_W2, grad_b2, B, N, (cudaStream_t)stream, h1_saved, pair_inv_scale, grad_R);
 }
 
+AHV_API size_t ahv_score_backward_det_workspace_bytes(int B, int64_t N, int r_per_pair, int want_grad_R) {
+  if (B < 0 || !n_ok(N)) return 0;
+  return DetBwdWs(B, N, want_grad_R && !r_per_pair).total * sizeof(float);
+}
+
+AHV_API int ahv_score_backward_det(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
+                                   const float* W1, const float* W2, const float* b2, const float* base,
+                                   const float* grad_scores, const void* h1_saved, const float* pair_inv_scale,
+                                   float* grad_vol, float* grad_tgt, float* grad_W1, float* grad_W2, float* grad_b2,
+                                   float* grad_R, int B, int64_t N, int math_mode, void* workspace, size_t workspace_bytes,
+                                   void* stream) {
+  if (B < 0 || !n_ok(N)) return AHV_EINVAL;
+  if (math_mode != AHV_MATH_TC && math_mode != AHV_MATH_FP32) return AHV_EINVAL;
+  if (!grad_vol && !grad_tgt && !grad_W1 && !grad_W2 && !grad_b2 && !grad_R) return AHV_EINVAL;
+  if (math_mode == AHV_MATH_TC && (grad_R || !all_set(grad_vol, grad_tgt, grad_W1, grad_W2, grad_b2))) return AHV_EINVAL;
+  if (!h1_saved != !pair_inv_scale) return AHV_EINVAL;
+  if ((int64_t)B * N > 0 && !all_set(vol_src, tgt_feat, R, W1, W2, b2, base, grad_scores)) return AHV_EINVAL;
+  if (!all_aligned16(vol_src, tgt_feat, R, W1, W2, h1_saved, workspace)) return AHV_EINVAL;
+  const DetBwdWs w(B, N, grad_R && !r_per_pair);
+  if ((int64_t)B * N > 0 && (!workspace || workspace_bytes < w.total * sizeof(float))) return AHV_EWORKSPACE;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  return launch_score_bwd_det(vol_src, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, grad_scores, h1_saved,
+                              pair_inv_scale, grad_vol, grad_tgt, grad_W1, grad_W2, grad_b2, grad_R, B, N,
+                              h1_saved && math_mode == AHV_MATH_TC, static_cast<float*>(workspace), (cudaStream_t)stream);
+}
+
 AHV_API int ahv_infonce(const float* scores, const float* R, int r_per_pair, const float* gt_R, float acc_thr_deg,
                         float temperature, float* loss, float* grad_scores, int B, int64_t N, void* stream) {
   if (B < 0 || N < 1 || !(temperature > 0.0f)) return AHV_EINVAL;

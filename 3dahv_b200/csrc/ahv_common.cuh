@@ -120,6 +120,43 @@ __device__ __forceinline__ float key_score(u64 key) {
 }
 __device__ __forceinline__ uint32_t key_index(u64 key) { return 0xFFFFFFFFu - (uint32_t)key; }
 
+// Ascending sort of a[0 .. kM) in registers (kM <= kN, kN a power of two; a[kM .. kN) hold 0xffffffff): Batcher's
+// odd-even merge network for kN inputs, fully unrolled, without the comparators that touch a place >= kM.  Every
+// comparator puts the smaller value at the lower place, so those places keep the largest value and their comparators
+// are no-ops.  19, 42 and 63 comparators for (8, 8), (16, 12) and (16, 16) (each checked on all 0-1 inputs).
+template <int kN, int kM>
+__device__ __forceinline__ void oddeven_sort(uint32_t* a) {
+#pragma unroll
+  for (int p = 1; p < kN; p <<= 1)
+#pragma unroll
+    for (int k = p; k >= 1; k >>= 1)
+#pragma unroll
+      for (int x = 0; x < kN; ++x)   // comparator (x, x + k): x = j + i, j = k % p (mod 2k), i < k, same 2p-block
+        if (x + k < kM && x >= k % p && (x - k % p) % (2 * k) < k && x / (2 * p) == (x + k) / (2 * p)) {
+          const uint32_t lo = min(a[x], a[x + k]);
+          a[x + k] = max(a[x], a[x + k]);
+          a[x] = lo;
+        }
+}
+// the n <= 16 register values of a warp whose largest count is nmax (warp-uniform)
+__device__ __forceinline__ void sort_row(uint32_t* a, int nmax) {
+  if (nmax <= 8) oddeven_sort<8, 8>(a);
+  else if (nmax <= 12) oddeven_sort<16, 12>(a);
+  else oddeven_sort<16, 16>(a);
+}
+
+// Insertion sort of one adjoint work list (offset of dX[vo], weight) by offset, which is unique per output voxel vo:
+// the deterministic backward sums every input voxel's contributions in this order, not in the order shared-memory
+// atomics handed out the places.  A rotation puts about 8 (at most ~12) entries on a voxel.
+__device__ __forceinline__ void sort_list(uint2* e, int n) {
+  for (int i = 1; i < n; ++i) {
+    const uint2 x = e[i];
+    int k = i;
+    for (; k > 0 && e[k - 1].x > x.x; --k) e[k] = e[k - 1];
+    e[k] = x;
+  }
+}
+
 
 namespace peer { struct Args; }  // ahv_peer.cuh
 
@@ -144,6 +181,33 @@ int launch_score_bwd_tc(const float* vol_src, const float* tgt_feat, const float
                         const float* W1, const float* W2, const float* b2, const float* base,
                         const float* grad_scores, const void* h1_saved, const float* pair_inv, float* g_vol,
                         float* g_tgt, float* g_W1, float* g_W2, float* g_b2, int B, int64_t N, cudaStream_t s);
+// Deterministic backward (ahv_score_backward_det).  The kernels store what the atomic instances add into global memory
+// in per-CTA workspace slots, and score_bwd_det_reduce adds the slots of every output element in increasing slot order.
+//   weight slot c (one per CTA, c < grid):   dW1 [32][384] | dW2 [32][32] | db2 [32]              kDetWSlot floats
+//   segment slot c + b (CTA c, pair b):     dV_b [16][512] | dT_b [32][64]                         kDetSegSlot floats
+// CTA c's items are contiguous, so c + b strictly increases over its segments: grid + B - 1 segment slots.
+// grid = min(B*N, SMs, kDetGridCap): the bits depend on the inputs and on min(SMs, kDetGridCap) alone, and the
+// workspace size on (B, N) alone.
+constexpr int kDetGridCap = 160;
+constexpr int kDetWSlot = kO * kK + kO * kO + kO;
+constexpr int kDetSegSlot = kC * kVox + kO * kP;
+struct DetBwdWs {   // offsets into the workspace in floats (each region 128-byte aligned); total * 4 bytes in all
+  int grid_max;
+  size_t seg, rot, total;   // rot: grad_R of every item [B*N][9] for a shared R (its sum over pairs)
+  DetBwdWs(int B, int64_t N, bool shared_grad_R)
+      : grid_max((int)((int64_t)B * N < kDetGridCap ? (int64_t)B * N : kDetGridCap)),
+        seg((size_t)grid_max * kDetWSlot),
+        rot(seg + (B > 0 && grid_max > 0 ? (size_t)(grid_max + B - 1) * kDetSegSlot : 0)),
+        total(rot + (shared_grad_R ? ((size_t)B * (size_t)N * 9 + 63) / 64 * 64 : 0)) {}
+};
+int launch_score_bwd_det(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
+                         const float* W1, const float* W2, const float* b2, const float* base, const float* grad_scores,
+                         const void* h1_saved, const float* pair_inv, float* g_vol, float* g_tgt, float* g_W1,
+                         float* g_W2, float* g_b2, float* g_R, int B, int64_t N, bool tc, float* ws, cudaStream_t s);
+int launch_score_bwd_tc_det(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
+                            const float* W1, const float* W2, const float* b2, const float* base,
+                            const float* grad_scores, const void* h1_saved, const float* pair_inv, float* ws_w,
+                            float* ws_seg, int B, int64_t N, unsigned grid, cudaStream_t s);
 int launch_score_tc_train(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair, const float* W1,
                           const float* W2, const float* b2, const float* base, float* scores, void* h1_out,
                           float* pair_inv_out, int B, int64_t N, void* ws, size_t ws_bytes, cudaStream_t s);

@@ -53,7 +53,10 @@ __device__ __forceinline__ int adjoint_out_voxel(int t, int j) {
 // kEx (ahv_score_backward_ex): every gradient output may be NULL - its accumulation and, for g_vol / g_W1 / g_R, its
 // phase are skipped - and the rotation-gradient phase (dS/dR into g_R) is compiled in.  kEx = false is the plain
 // backward of ahv_score_backward / ahv_score_backward_saved, which writes all five.
-template <bool kEx>
+// kDet (ahv_score_backward_det): no float atomics.  g_W1 / g_W2 / g_b2 point at the weight slots and g_vol / g_tgt at
+// the segment slots of the workspace (DetBwdWs, ahv_common.cuh), g_R at [B*N][9] for a shared R; every input voxel's
+// adjoint list is summed in increasing output-voxel order.
+template <bool kEx, bool kDet>
 __global__ void __launch_bounds__(kThreads, 1)
 score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tgt_feat,
                  const float* __restrict__ R, int r_per_pair, const float* __restrict__ W1,
@@ -96,6 +99,21 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
     for (int c = 0; c < kC; ++c) aV[j][c] = 0.0f;
 
   auto flush_pair = [&](int b) {  // dT and dV of pair b leave the CTA
+    if constexpr (kDet) {   // the whole segment, zeros included, into slot blockIdx.x + b
+      const size_t slot = (size_t)(blockIdx.x + b) * kDetSegSlot;
+#pragma unroll
+      for (int oo = 0; oo < 8; ++oo) {
+        if (want_tgt) g_tgt[slot + (cg2 * 8 + oo) * kP + pos] = aT[oo];
+        aT[oo] = 0.0f;
+      }
+#pragma unroll
+      for (int j = 0; j < 2; ++j)
+#pragma unroll
+        for (int c = 0; c < kC; ++c) {
+          if (want_vol) g_vol[slot + c * kVox + t + 256 * j] = aV[j][c];
+          aV[j][c] = 0.0f;
+        }
+    } else {
 #pragma unroll
     for (int oo = 0; oo < 8; ++oo) {
       if (want_tgt && aT[oo] != 0.0f) atomicAdd(g_tgt + ((size_t)b * kO + cg2 * 8 + oo) * kP + pos, aT[oo]);
@@ -108,6 +126,7 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
         if (want_vol && aV[j][c] != 0.0f) atomicAdd(g_vol + ((size_t)b * kC + c) * kVox + t + 256 * j, aV[j][c]);
         aV[j][c] = 0.0f;
       }
+    }
   };
 
   int cur_b = -1;
@@ -210,6 +229,7 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
       const float sR = rotation_grad(sm, bs.dh2 + 2 * kVox, t);
       if (t < 9) {
         if (r_per_pair) g_R[(size_t)it * 9 + t] += sR;   // the item is this CTA's alone
+        else if constexpr (kDet) g_R[(size_t)it * 9 + t] = sR;   // summed over the pairs by score_bwd_det_reduce
         else atomicAdd(g_R + (size_t)n * 9 + t, sR);
       }
     }
@@ -287,6 +307,55 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
           }
       }
       __syncthreads();
+      if constexpr (kDet) {
+        // The atomics ranked each list in arrival order; it is summed in increasing dX offset instead.  Up to 16 entries
+        // (a rotation puts at most ~12 on a voxel) the keys (offset, place) are sorted in registers by a network and the
+        // entries read in that order; longer lists (matrices that crowd the samples) are sorted in place first.
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+          const int vi = t + 256 * j;
+          const int nn = cnt[vi];
+          uint2* e = ent + start[vi];
+          int nmax = nn;
+#pragma unroll
+          for (int o = 16; o > 0; o >>= 1) nmax = max(nmax, __shfl_xor_sync(0xffffffffu, nmax, o));
+          if (nmax <= 16) {
+            uint32_t key[16];
+#pragma unroll
+            for (int i = 0; i < 16; ++i) key[i] = i < nn ? (e[i].x << 4) | (uint32_t)i : 0xffffffffu;
+            sort_row(key, nmax);
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+              if (i >= nmax) break;   // warp-uniform
+              if (i < nn) {
+                const uint2 en = e[key[i] & 15u];
+                const float w = __uint_as_float(en.y);
+                const float* src = sm.rotA + en.x;
+#pragma unroll
+                for (int c4 = 0; c4 < 4; ++c4) {
+                  const float4 x = *reinterpret_cast<const float4*>(src + 4 * c4);
+                  aV[j][4 * c4] = fmaf(w, x.x, aV[j][4 * c4]); aV[j][4 * c4 + 1] = fmaf(w, x.y, aV[j][4 * c4 + 1]);
+                  aV[j][4 * c4 + 2] = fmaf(w, x.z, aV[j][4 * c4 + 2]); aV[j][4 * c4 + 3] = fmaf(w, x.w, aV[j][4 * c4 + 3]);
+                }
+              }
+            }
+            continue;
+          }
+          sort_list(e, nn);
+#pragma unroll 2
+          for (int i = 0; i < nn; ++i) {
+            const uint2 en = e[i];
+            const float w = __uint_as_float(en.y);
+            const float* src = sm.rotA + en.x;
+#pragma unroll
+            for (int c4 = 0; c4 < 4; ++c4) {
+              const float4 x = *reinterpret_cast<const float4*>(src + 4 * c4);
+              aV[j][4 * c4] = fmaf(w, x.x, aV[j][4 * c4]); aV[j][4 * c4 + 1] = fmaf(w, x.y, aV[j][4 * c4 + 1]);
+              aV[j][4 * c4 + 2] = fmaf(w, x.z, aV[j][4 * c4 + 2]); aV[j][4 * c4 + 3] = fmaf(w, x.w, aV[j][4 * c4 + 3]);
+            }
+          }
+        }
+      } else {
 #pragma unroll
       for (int j = 0; j < 2; ++j) {
         const int vi = t + 256 * j;
@@ -305,6 +374,7 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
           }
         }
       }
+      }
     }
     __syncthreads();  // dX, the work list and the taps are re-used by the next hypothesis
   }
@@ -317,15 +387,23 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
 #pragma unroll
       for (int kk = 0; kk < 8; ++kk) {
         const int k = view * 128 + c * 8 + kk;
-        if (want_W1) {
+        if constexpr (kDet) {
+          if (want_W1) {
+            g_W1[(size_t)blockIdx.x * kDetWSlot + (2 * cg) * kK + k] = aW1[view][kk][0];
+            g_W1[(size_t)blockIdx.x * kDetWSlot + (2 * cg + 1) * kK + k] = aW1[view][kk][1];
+          }
+        } else if (want_W1) {
           atomicAdd(g_W1 + (2 * cg) * kK + k, aW1[view][kk][0]);
           atomicAdd(g_W1 + (2 * cg + 1) * kK + k, aW1[view][kk][1]);
         }
       }
     const int o = t >> 3, i0 = (t & 7) * 4;
 #pragma unroll
-    for (int i = 0; i < 4; ++i)
-      if (want_W2) atomicAdd(g_W2 + o * kO + i0 + i, aW2[i]);
+    for (int i = 0; i < 4; ++i) {
+      if constexpr (kDet) {
+        if (want_W2) g_W2[(size_t)blockIdx.x * kDetWSlot + o * kO + i0 + i] = aW2[i];
+      } else if (want_W2) atomicAdd(g_W2 + o * kO + i0 + i, aW2[i]);
+    }
     // db2: sum over the 64 positions inside the CTA first (threads with equal cg2 = t & 3)
     __syncthreads();
     float* red = sm.h1s;  // [4 cg2][8 oo][64 pos]
@@ -335,7 +413,8 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
     if (want_b2 && t < kO) {
       float s = 0.0f;
       for (int p = 0; p < kP; ++p) s += red[t * kP + p];
-      atomicAdd(g_b2 + t, s);
+      if constexpr (kDet) g_b2[(size_t)blockIdx.x * kDetWSlot + t] = s;
+      else atomicAdd(g_b2 + t, s);
     }
   }
 }
@@ -354,14 +433,113 @@ int launch_score_bwd(const float* vol_src, const float* tgt_feat, const float* R
   const size_t smem = sizeof(BwdSmem);
   const __half* h1 = static_cast<const __half*>(h1_saved);
   if (g_R || !g_vol || !g_tgt || !g_W1 || !g_W2 || !g_b2) {
-    AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    score_bwd_kernel<true><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
+    AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    score_bwd_kernel<true, false><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
                                                         g_vol, g_tgt, g_W1, g_W2, g_b2, B, N, h1, pair_inv, g_R);
   } else {
-    AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    score_bwd_kernel<false><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
+    AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    score_bwd_kernel<false, false><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
                                                          g_vol, g_tgt, g_W1, g_W2, g_b2, B, N, h1, pair_inv, nullptr);
   }
+  AHV_CUDA_OK(cudaGetLastError());
+  return AHV_OK;
+}
+
+// Largest CTA c of a grid over `total` items whose first item, total * c / grid, is at or before item i.
+__device__ __forceinline__ int cta_of(int64_t i, int64_t total, int grid) {
+  int c = (int)(i * grid / total);
+  while (c + 1 < grid && total * (c + 1) / grid <= i) ++c;
+  return c;
+}
+
+// The deterministic backward's fixed-order reduction: one thread per output element adds the element's partials in
+// increasing slot order - the weight slots of CTAs 0 .. grid-1, the segment slots c + b of the CTAs c that hold items of
+// pair b, a shared R's per-item values over b = 0 .. B-1 - and adds the sum into the output with one plain add.
+// Index space: [W1 | W2 | b2] (kDetWSlot), then B segments [dV_b | dT_b] (kDetSegSlot each), then grad_R [N][9] when a
+// shared R's gradient is asked for.  NULL outputs are skipped.
+__global__ void __launch_bounds__(256)
+score_bwd_det_reduce(const float* __restrict__ ws, size_t seg_off, size_t rot_off, int grid, int B, int64_t N,
+                     float* __restrict__ g_vol, float* __restrict__ g_tgt, float* __restrict__ g_W1,
+                     float* __restrict__ g_W2, float* __restrict__ g_b2, float* __restrict__ g_R_shared) {
+  const int64_t total = (int64_t)B * N;
+  const int64_t n_w = kDetWSlot, n_seg = (int64_t)B * kDetSegSlot, n_all = n_w + n_seg + (g_R_shared ? N * 9 : 0);
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n_all; i += (int64_t)gridDim.x * blockDim.x) {
+    if (i < n_w) {
+      const int e = (int)i;
+      float* out = e < kO * kK ? (g_W1 ? g_W1 + e : nullptr)
+                 : e < kO * kK + kO * kO ? (g_W2 ? g_W2 + (e - kO * kK) : nullptr)
+                 : (g_b2 ? g_b2 + (e - kO * kK - kO * kO) : nullptr);
+      if (!out) continue;
+      float s = ws[e];
+      for (int c = 1; c < grid; ++c) s += ws[(size_t)c * kDetWSlot + e];
+      *out += s;
+    } else if (i < n_w + n_seg) {
+      const int64_t j = i - n_w;
+      const int b = (int)(j / kDetSegSlot), f = (int)(j - (int64_t)b * kDetSegSlot);
+      float* out = f < kC * kVox ? (g_vol ? g_vol + (size_t)b * kC * kVox + f : nullptr)
+                                 : (g_tgt ? g_tgt + (size_t)b * kO * kP + (f - kC * kVox) : nullptr);
+      if (!out) continue;
+      const int c0 = cta_of((int64_t)b * N, total, grid), c1 = cta_of((int64_t)(b + 1) * N - 1, total, grid);
+      const float* p = ws + seg_off + f;
+      float s = p[(size_t)(c0 + b) * kDetSegSlot];
+      for (int c = c0 + 1; c <= c1; ++c) s += p[(size_t)(c + b) * kDetSegSlot];
+      *out += s;
+    } else {
+      const int64_t j = i - n_w - n_seg;   // n * 9 + e
+      const float* p = ws + rot_off + j;
+      float s = p[0];
+      for (int b = 1; b < B; ++b) s += p[(size_t)b * N * 9];
+      g_R_shared[j] += s;
+    }
+  }
+}
+
+int launch_score_bwd_det(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
+                         const float* W1, const float* W2, const float* b2, const float* base, const float* grad_scores,
+                         const void* h1_saved, const float* pair_inv, float* g_vol, float* g_tgt, float* g_W1,
+                         float* g_W2, float* g_b2, float* g_R, int B, int64_t N, bool tc, float* ws, cudaStream_t s) {
+  const int64_t total = (int64_t)B * N;
+  if (total == 0) return AHV_OK;
+  int dev = 0, sms = 0;
+  AHV_CUDA_OK(cudaGetDevice(&dev));
+  AHV_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  const int grid = (int)std::min<int64_t>(total, std::min(sms, kDetGridCap));
+  const bool shared_R = g_R && !r_per_pair;
+  const DetBwdWs w(B, N, shared_R);
+  float* ws_w = ws;
+  float* ws_seg = ws + w.seg;
+  if (tc) {
+    const int st = launch_score_bwd_tc_det(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores, h1_saved,
+                                           pair_inv, ws_w, ws_seg, B, N, (unsigned)grid, s);
+    if (st != AHV_OK) return st;
+  } else {
+    // the kernel's outputs are the workspace slots (NULL where the caller's output is NULL); a per-pair R's gradient
+    // has one writer per element and goes straight to the caller's buffer
+    float* k_vol = g_vol ? ws_seg : nullptr;
+    float* k_tgt = g_tgt ? ws_seg + kC * kVox : nullptr;
+    float* k_W1 = g_W1 ? ws_w : nullptr;
+    float* k_W2 = g_W2 ? ws_w + kO * kK : nullptr;
+    float* k_b2 = g_b2 ? ws_w + kO * kK + kO * kO : nullptr;
+    float* k_R = g_R ? (r_per_pair ? g_R : ws + w.rot) : nullptr;
+    const size_t smem = sizeof(BwdSmem);
+    const __half* h1 = static_cast<const __half*>(h1_saved);
+    if (g_R || !g_vol || !g_tgt || !g_W1 || !g_W2 || !g_b2) {
+      AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      score_bwd_kernel<true, true><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base,
+                                                                grad_scores, k_vol, k_tgt, k_W1, k_W2, k_b2, B, N, h1,
+                                                                pair_inv, k_R);
+    } else {
+      AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      score_bwd_kernel<false, true><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base,
+                                                                 grad_scores, k_vol, k_tgt, k_W1, k_W2, k_b2, B, N, h1,
+                                                                 pair_inv, nullptr);
+    }
+    AHV_CUDA_OK(cudaGetLastError());
+  }
+  const int64_t n_all = kDetWSlot + (int64_t)B * kDetSegSlot + (shared_R ? N * 9 : 0);
+  const unsigned blocks = (unsigned)std::min<int64_t>((n_all + 255) / 256, 8 * (int64_t)sms);
+  score_bwd_det_reduce<<<blocks, 256, 0, s>>>(ws, w.seg, w.rot, grid, B, N, g_vol, g_tgt, g_W1, g_W2, g_b2,
+                                              shared_R ? g_R : nullptr);
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }

@@ -42,6 +42,11 @@
 //
 // Gradients are those of the function the tensor-core forward evaluated (its ReLU mask), with fp16 operand rounding:
 // checked to 1e-3 of each gradient's maximum against fp64 autograd of that function (tests/test_gpu_training.py).
+//
+// kDet (ahv_score_backward_det): no float atomics - dV, dT and the weight gradients go to the workspace slots of
+// DetBwdWs (ahv_common.cuh: g_vol / g_tgt point at the segment slots, g_W1 / g_W2 / g_b2 at the weight slots) - and
+// every input voxel's contributions are summed in increasing output-voxel order: a sorting network over the row in
+// registers (oddeven_sort), an insertion sort of the exact path's lists.
 #include <cstddef>
 
 #include "ahv_head_fp32.cuh"
@@ -227,6 +232,7 @@ __device__ __forceinline__ void pack_views(BwdTcSmem& sm, float sb) {
   }
 }
 
+template <bool kDet>
 __global__ void __launch_bounds__(kThreads, 1)
 score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__ tgt_feat,
                     const float* __restrict__ R, int r_per_pair, const float* __restrict__ W1,
@@ -349,6 +355,21 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
     for (int c = 0; c < kC; ++c) aV[j][c] = 0.0f;
 
   auto flush_pair = [&](int b) {  // dT and dV of pair b leave the CTA
+    if constexpr (kDet) {   // the whole segment, zeros included, into slot blockIdx.x + b
+      const size_t slot = (size_t)(blockIdx.x + b) * kDetSegSlot;
+#pragma unroll
+      for (int oo = 0; oo < 8; ++oo) {
+        g_tgt[slot + (cg2 * 8 + oo) * kP + pos] = aT[oo];
+        aT[oo] = 0.0f;
+      }
+#pragma unroll
+      for (int j = 0; j < 2; ++j)
+#pragma unroll
+        for (int c = 0; c < kC; ++c) {
+          g_vol[slot + c * kVox + t + 256 * j] = aV[j][c];
+          aV[j][c] = 0.0f;
+        }
+    } else {
 #pragma unroll
     for (int oo = 0; oo < 8; ++oo) {
       if (aT[oo] != 0.0f) atomicAdd(g_tgt + ((size_t)b * kO + cg2 * 8 + oo) * kP + pos, aT[oo]);
@@ -361,6 +382,7 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
         if (aV[j][c] != 0.0f) atomicAdd(g_vol + ((size_t)b * kC + c) * kVox + t + 256 * j, aV[j][c]);
         aV[j][c] = 0.0f;
       }
+    }
   };
 
   // ---- the adjoint's work list ----
@@ -700,12 +722,25 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
             en[4 * q] = x.x; en[4 * q + 1] = x.y; en[4 * q + 2] = x.z; en[4 * q + 3] = x.w;
           }
         }
+        if constexpr (kDet) {
+          // the row in increasing record offset: halves swapped (offset on top, unique per output voxel), the unused
+          // places above every entry; the network's size follows the warp's longest row
+#pragma unroll
+          for (int i = 0; i < kListCap; ++i) en[i] = i < nn ? __byte_perm(en[i], 0, 0x1032) : 0xffffffffu;
+          sort_row(en, nmax);
+#pragma unroll
+          for (int i = 0; i < kListCap; ++i) {
+            if (i >= nmax) break;   // warp-uniform
+            if (i < nn) axpy_record(aV[j], (float)(en[i] & 0xffffu) * wq, dX + ((en[i] >> 16) << 2));
+          }
+        } else {
 #pragma unroll
         for (int i = 0; i < kListCap; ++i) {
           if (i >= nmax) break;   // warp-uniform
           if (i < nn) {
             axpy_record(aV[j], (float)(en[i] >> 16) * wq, dX + ((en[i] & 0xffffu) << 2));
           }
+        }
         }
       }
     } else {
@@ -776,6 +811,10 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
         }
       }
       __syncthreads();
+      if constexpr (kDet) {   // the atomics ranked each list in arrival order: sort the thread's two lists by dX offset
+#pragma unroll
+        for (int j = 0; j < 2; ++j) sort_list(ent + start[t + 256 * j], cnt[t + 256 * j]);
+      }
 #pragma unroll
       for (int j = 0; j < 2; ++j) {
         const int vi = t + 256 * j;
@@ -804,15 +843,24 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
   }
 #endif
   flush_pair(cur_b);
-  // weight gradients: one atomic per accumulator and CTA
+  // weight gradients: one atomic per accumulator and CTA (kDet: one store into the CTA's weight slot)
+  const size_t wslot = kDet ? (size_t)blockIdx.x * kDetWSlot : 0;
 #pragma unroll
   for (int view = 0; view < 3; ++view)
 #pragma unroll
-    for (int oo = 0; oo < 16; ++oo) atomicAdd(g_W1 + (16 * hf + oo) * kK + view * 128 + 32 * qd + lane, aW1[view][oo]);
+    for (int oo = 0; oo < 16; ++oo) {
+      float* dst = g_W1 + wslot + (16 * hf + oo) * kK + view * 128 + 32 * qd + lane;
+      if constexpr (kDet) *dst = aW1[view][oo];
+      else atomicAdd(dst, aW1[view][oo]);
+    }
   {
     if (qd < 2) {
 #pragma unroll
-      for (int i = 0; i < 8; ++i) atomicAdd(g_W2 + (16 * qd + (lane & 15)) * kO + 16 * (lane >> 4) + 8 * hf + i, aW2[i]);
+      for (int i = 0; i < 8; ++i) {
+        float* dst = g_W2 + wslot + (16 * qd + (lane & 15)) * kO + 16 * (lane >> 4) + 8 * hf + i;
+        if constexpr (kDet) *dst = aW2[i];
+        else atomicAdd(dst, aW2[i]);
+      }
     }
     // db2: sum over the 64 positions inside the CTA first (threads with equal cg2 = t & 3)
     __syncthreads();
@@ -823,7 +871,8 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
     if (t < kO) {
       float s = 0.0f;
       for (int p = 0; p < kP; ++p) s += red[t * kP + p];
-      atomicAdd(g_b2 + t, s);
+      if constexpr (kDet) g_b2[wslot + t] = s;
+      else atomicAdd(g_b2 + t, s);
     }
   }
   tc_fence_before();
@@ -848,10 +897,26 @@ int launch_score_bwd_tc(const float* vol_src, const float* tgt_feat, const float
   AHV_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   const unsigned grid = (unsigned)(total < sms ? total : sms);
   const size_t smem = sizeof(BwdTcSmem);
-  AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  score_bwd_tc_kernel<<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
+  AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  score_bwd_tc_kernel<false><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
                                                    static_cast<const __half*>(h1_saved), pair_inv, g_vol, g_tgt,
                                                    g_W1, g_W2, g_b2, B, N);
+  AHV_CUDA_OK(cudaGetLastError());
+  return AHV_OK;
+}
+
+// the kDet instance on `grid` CTAs (launch_score_bwd_det picks it and reduces the slots)
+int launch_score_bwd_tc_det(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
+                            const float* W1, const float* W2, const float* b2, const float* base,
+                            const float* grad_scores, const void* h1_saved, const float* pair_inv, float* ws_w,
+                            float* ws_seg, int B, int64_t N, unsigned grid, cudaStream_t s) {
+  if (!h1_saved || !pair_inv) return AHV_EINVAL;
+  const size_t smem = sizeof(BwdTcSmem);
+  AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  score_bwd_tc_kernel<true><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
+                                                         static_cast<const __half*>(h1_saved), pair_inv, ws_seg,
+                                                         ws_seg + kC * kVox, ws_w, ws_w + kO * kK, ws_w + kO * kK + kO * kO,
+                                                         B, N);
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }

@@ -206,7 +206,8 @@ def _score_backward_args(vol_src, tgt_feat, R, W1, W2, b2, grad_scores):
 
 def score_backward(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tensor, W1: torch.Tensor, W2: torch.Tensor,
                    b2: torch.Tensor, grad_scores: torch.Tensor, h1_saved: torch.Tensor | None = None,
-                   pair_inv: torch.Tensor | None = None, math: int = MATH_TC, want_grad_R: bool = False):
+                   pair_inv: torch.Tensor | None = None, math: int = MATH_TC, want_grad_R: bool = False,
+                   deterministic: bool = False, workspace: torch.Tensor | None = None):
     """Fused gradient of the verification scores (modules/model.py:53-56 under autograd): returns
     (grad_vol_src [B,16,8,8,8], grad_tgt_feat [B,32,64], grad_W1 [32,384], grad_W2 [32,32], grad_b2 [32]).
     With `h1_saved` / `pair_inv` from `score_train` the kernel reads conv1's output instead of recomputing it, and
@@ -214,7 +215,12 @@ def score_backward(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tenso
     it is the exact fp32 kernel whatever `math` says.
     `want_grad_R`: also the gradient w.r.t. the rotations, appended to the tuple - grad_R [N,3,3] (summed over pairs)
     or [B,N,3,3] - from `ahv_score_backward_ex`, which contracts in fp32 FFMA whatever `math` says (the tcgen05
-    backward has no rotation phase; with saved activations this is the MATH_FP32 form on the same saved values)."""
+    backward has no rotation phase; with saved activations this is the MATH_FP32 form on the same saved values).
+    `deterministic`: the same kernels and routing, in the form of `ahv_score_backward_det`, which sums every gradient
+    in a fixed order instead of with float atomics: bit-identical results from run to run on one device (the bits
+    depend on the inputs and on min(SM count, 160)).  It needs `ahv_score_backward_det_workspace_bytes` of scratch,
+    about 15 MB at B = 12 (16 MB more with a shared R's gradient at N = 9000); `workspace` re-uses a buffer of at least
+    that size, else one is allocated."""
     vs, tg, R, W1, W2, b2, gs, B, N, per_pair = _score_backward_args(vol_src, tgt_feat, R, W1, W2, b2, grad_scores)
     dev = vs.device
     z = lambda *shape: torch.zeros(*shape, device=dev, dtype=torch.float32)
@@ -225,6 +231,17 @@ def score_backward(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tenso
         pi = _dev(pair_inv, "pair_inv")
         if h1.numel() != B * N * 64 * 32 or pi.numel() != B:
             raise ValueError("h1_saved [B*N,64,32] fp16 and pair_inv [B] expected")
+    if deterministic:
+        g_R = z(*R.shape) if want_grad_R else None
+        outs = (g_vol, g_tgt, g_w1, g_w2, g_b2, g_R)
+        mode = int(math) if h1 is not None and not want_grad_R else MATH_FP32
+        need = score_backward_det_workspace_bytes(B, N, per_pair, want_grad_R)
+        workspace, ws_bytes = _workspace(workspace, need, dev)
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        _call("ahv_score_backward_det", dev, vs.data_ptr(), tg.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(),
+              W2.data_ptr(), b2.data_ptr(), base_coords(dev).data_ptr(), gs.data_ptr(), ptr(h1), ptr(pi),
+              *(ptr(t) for t in outs), B, N, mode, workspace.data_ptr(), ws_bytes)
+        return outs if want_grad_R else outs[:5]
     if want_grad_R:
         g_R = z(*R.shape)
         _score_backward_ex(vs, tg, R, W1, W2, b2, gs, h1, pi, (g_vol, g_tgt, g_w1, g_w2, g_b2, g_R), B, N, per_pair)
@@ -237,6 +254,11 @@ def score_backward(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tenso
     else:
         _call("ahv_score_backward", dev, *head, *tail)
     return g_vol, g_tgt, g_w1, g_w2, g_b2
+
+
+def score_backward_det_workspace_bytes(B: int, N: int, per_pair: bool, want_grad_R: bool) -> int:
+    """Bytes of scratch `score_backward(..., deterministic=True)` needs (0 for invalid sizes)."""
+    return int(_lib.lib().ahv_score_backward_det_workspace_bytes(B, N, int(per_pair), int(want_grad_R)))
 
 
 def score_grad_R(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tensor, W1: torch.Tensor, W2: torch.Tensor,

@@ -17,8 +17,14 @@ Arithmetic: with the default `math=MATH_TC` the FORWARD scores carry the tensor-
 (~1e-4 relative) while the fused backward recomputes the forward in fp32, i.e. the gradient is that of a function
 1e-4 away from the loss reported (tests/test_gpu_training.py holds the end-to-end gradients to 5e-3 of their maximum
 against the reference's autograd in this mode, 2e-4 with `math=MATH_FP32`, which is 8x slower in the forward only).
-The backward accumulates dV, dT, dW1, dW2, db2 across CTAs with float atomics, so gradients are reproducible to
-rounding, not bit for bit, from run to run.
+By default the backward accumulates dV, dT, dW1, dW2, db2 across CTAs with float atomics, so gradients are
+reproducible to rounding, not bit for bit, from run to run.  Under `torch.use_deterministic_algorithms(True)` (read when
+the backward runs, as PyTorch's own ops do; Lightning's `Trainer(deterministic=True)` sets it) the fused backward runs
+the deterministic form of the same kernels instead (`ahv_score_backward_det`: per-CTA partials in a workspace, summed
+in a fixed order), and gradients are bit-identical from run to run on one device.  The paths that still scatter with
+float atomics - `rotate_volume`'s backward w.r.t. the volume (`ahv_rotate_volume_backward`), and so
+`fused_backward=False` - then follow PyTorch's convention for `F.grid_sample`'s backward: they raise a RuntimeError
+naming the op, or warn under `warn_only=True`.
 
 Fast form (`save_activations=True`, opt-in): the tensor-core forward also keeps conv1's ReLU'd output (fp16, 4 KB per
 hypothesis - `ahv_score_train`), and the backward (`ahv_score_backward_saved`, csrc/ahv_score_bwd_tc.cu) reads it
@@ -35,12 +41,28 @@ ATen's convention at lattice points and at the volume's edge (DESIGN.md §4.4). 
 from __future__ import annotations
 
 import math
+import warnings
 
 import torch
 import torch.nn.functional as F
 
 from . import ops
 from ._lib import MATH_FP32, MATH_TC
+
+
+def _alert_not_deterministic(op: str) -> None:
+    """PyTorch's convention for an op without a deterministic implementation under
+    `torch.use_deterministic_algorithms(True)`: raise, or warn with `warn_only=True`."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return
+    msg = (f"{op} does not have a deterministic implementation, but you set 'torch.use_deterministic_algorithms(True)'. "
+           "You can turn off determinism just for this operation, or you can use the 'warn_only=True' option, if that's "
+           "acceptable for your application. verification_scores with fused_backward=True (the default) has a "
+           "deterministic backward.")
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        warnings.warn(msg, UserWarning, stacklevel=3)
+    else:
+        raise RuntimeError(msg)
 
 
 class _RotateVolume(torch.autograd.Function):
@@ -57,6 +79,8 @@ class _RotateVolume(torch.autograd.Function):
     def backward(ctx, grad_out):
         R, volume = ctx.saved_tensors
         g = grad_out.contiguous()
+        if ctx.needs_input_grad[0]:   # the adjoint scatters with float atomics; the gradient w.r.t. R has one writer
+            _alert_not_deterministic("ahv_rotate_volume_backward (the backward of training.rotate_volume w.r.t. the volume)")
         g_vol = ops.rotate_volume_backward(g, R, ctx.per_rot) if ctx.needs_input_grad[0] else None
         g_R = ops.rotate_volume_grad_R(volume, g, R, ctx.per_rot) if ctx.needs_input_grad[1] else None
         return g_vol, g_R
@@ -115,7 +139,7 @@ class _VerifyScores(torch.autograd.Function):
             # values and ReLU mask) plus its rotation phase - the tcgen05 backward has none
             g = ops.score_backward(vol_src.detach().float(), tgt_saved, R.detach(), W1.detach().float(), W2.detach().float(),
                                    b2.detach().float(), grad_scores.contiguous().float(), h1, pair_inv, ctx.bwd_math,
-                                   want_grad_R=want_R)
+                                   want_grad_R=want_R, deterministic=torch.are_deterministic_algorithms_enabled())
             g_vs, g_tgt, g_w1, g_w2, g_b = g[:5]
             with torch.enable_grad():   # target side: B volumes through the differentiable head
                 vt = vol_tgt.detach().float().requires_grad_(True)
@@ -168,7 +192,10 @@ def verification_scores(vol_src, vol_tgt, R, W1, W2, b2, math: int = MATH_TC, ch
     When `R` requires a gradient, `R.grad` is d/dR of the scores ([N,3,3] summed over pairs, or [B,N,3,3]).  The fused
     backward computes it, and the other gradients, with `ahv_score_backward_ex` in fp32 FFMA; with saved activations
     that call replaces the tcgen05 backward whatever `tc_backward` says (same kept values, same ReLU mask, fp32
-    contractions).  The chunked form differentiates through `rotate_volume` instead."""
+    contractions).  The chunked form differentiates through `rotate_volume` instead.
+    Under `torch.use_deterministic_algorithms(True)` the fused backward runs the deterministic form of whichever kernel
+    the rules above pick (`ops.score_backward(..., deterministic=True)`): bit-identical gradients from run to run.  The
+    chunked form (`fused_backward=False`) has none: it raises there, or warns with `warn_only=True`."""
     return _VerifyScores.apply(vol_src, vol_tgt, R.contiguous(), W1, W2, b2, math, chunk, fused_backward, save_activations,
                                tc_backward)
 

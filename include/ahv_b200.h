@@ -180,6 +180,28 @@ AHV_API int ahv_score_backward_ex(const float* vol_src, const float* tgt_feat, c
                                   float* grad_vol, float* grad_tgt, float* grad_W1, float* grad_W2, float* grad_b2,
                                   float* grad_R, int B, int64_t N, void* stream);
 
+/* Deterministic form of the three backward entries above: bit-identical gradients from run to run (what PyTorch's
+ * torch.use_deterministic_algorithms asks for).  Arguments as ahv_score_backward_ex, plus:
+ *   math_mode   AHV_MATH_FP32 or AHV_MATH_TC.  h1_saved/pair_inv_scale NULL = the recompute form (fp32 FFMA, as
+ *               ahv_score_backward / _ex); with them, AHV_MATH_FP32 = the FFMA form and AHV_MATH_TC = the tcgen05 form
+ *               of ahv_score_backward_saved.  AHV_MATH_TC needs all five of grad_vol .. grad_b2 and no grad_R.
+ *   workspace   ahv_score_backward_det_workspace_bytes(B, N, r_per_pair, grad_R != NULL) bytes, 16-byte aligned.
+ * Gradients are ADDED into the caller-zeroed outputs, as the other entries do, but no float atomics are used: each CTA
+ * stores its partials in its own workspace slots - the weight gradients in slot c (CTA c), dV and dT of pair b in slot
+ * c + b, a shared R's gradient per item - and a second kernel adds every output element's partials in increasing slot
+ * order, then adds the sum into the output.  Inside a CTA, every input voxel's share of the resampling adjoint is
+ * summed in increasing output-voxel order.  The grid is min(B*N, SMs, 160) CTAs, so the bits depend only on the
+ * inputs and on min(SMs, 160): two devices with at least 160 SMs, or with the same SM count, give the same bits.
+ * The function computed is that of the atomic entries; only the summation order differs (one-item calls run one CTA
+ * and give the same bits for everything but grad_vol).  Graph-capturable; allocates nothing. */
+AHV_API size_t ahv_score_backward_det_workspace_bytes(int B, int64_t N, int r_per_pair, int want_grad_R);
+AHV_API int ahv_score_backward_det(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
+                                   const float* W1, const float* W2, const float* b2, const float* base,
+                                   const float* grad_scores, const void* h1_saved, const float* pair_inv_scale,
+                                   float* grad_vol, float* grad_tgt, float* grad_W1, float* grad_W2, float* grad_b2,
+                                   float* grad_R, int B, int64_t N, int math_mode, void* workspace, size_t workspace_bytes,
+                                   void* stream);
+
 /* infoNCE_loss given the scores (training variant, modules/model.py:43-63 / model_co3d.py:41-61), one launch:
  * positives of pair b = hypotheses whose rotation lies within acc_thr_deg of gt_R[b] (:46-49);
  * loss[b] = -log(sum_pos exp(s/T) / max(sum_all exp(s/T), 1e-8)) (:58-61); grad_scores [B,N] (or NULL) receives
