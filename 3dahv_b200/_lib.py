@@ -68,6 +68,14 @@ SIGNATURES = {
                                _i, _i, _vp]),
     "ahv_verify_sharded": (_i, [_vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _i64, _i, _vp, _sz, _i, _i,
                                 ctypes.POINTER(ctypes.c_void_p), _i, _i, _vp]),
+    "ahv_peer_bytes_ex": (_sz, [_i, _i, _i64]),
+    "ahv_peer_alloc_ex": (_i, [_i, _i, _i64, ctypes.POINTER(ctypes.c_void_p)]),
+    "ahv_peer_capacity_ex": (_i, [_vp, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int64)]),
+    "ahv_scores_exchange": (_i, [_vp, _i, _i64, _vp, _i, _i, ctypes.POINTER(ctypes.c_void_p), _i, _i, _i64, _vp]),
+    "ahv_refine_gradient_sharded_workspace_bytes": (_sz, [_i, _i64, _i, _i]),
+    "ahv_refine_gradient_sharded": (_i, [_vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, ctypes.c_float, ctypes.c_float, _vp,
+                                         _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _vp, _sz, _i, _i,
+                                         ctypes.POINTER(ctypes.c_void_p), _i, _i, _i64, _vp]),
     "ahv_host_session_create": (_i, [ctypes.POINTER(ctypes.c_void_p)]),
     "ahv_host_session_destroy": (_i, [_vp]),
     "ahv_predict_host_ex": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _i64, _i, _i, _i,

@@ -1,5 +1,6 @@
 // extern "C" surface of lib3dahv_b200 (see include/ahv_b200.h for the contract
 // and the reference interface each entry replaces).
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <new>
@@ -58,6 +59,26 @@ struct RefineGradientWs {
         top(tgt + align_up((size_t)B * kO * kP * sizeof(float), 256)),
         total(top + align_up(topk_workspace_bytes(B, k, 1), 256)) {}
 };
+
+// ahv_refine_gradient_sharded (world > 1), per = ceil(N / world) hypotheses at most on a rank:
+// [the slice's verification workspace | the slice's rotations B*per*9 | the whole score matrix B*N (distinct pass 1)
+//  | target features B*32*64 | top-k partials over [B,k]]
+struct ShardedRefineWs {
+  size_t rs, full, tgt, top, total;
+  ShardedRefineWs(int B, int64_t N, int k, int world)
+      : rs(VerifyWs(B, (N + world - 1) / world, k).total),
+        full(rs + align_up((size_t)B * (size_t)((N + world - 1) / world) * 9 * sizeof(float), 256)),
+        tgt(full + align_up((size_t)B * (size_t)N * sizeof(float), 256)),
+        top(tgt + align_up((size_t)B * kO * kP * sizeof(float), 256)),
+        total(top + align_up(topk_workspace_bytes(B, k, 1), 256)) {}
+};
+
+// dist.shard_bounds: rank's contiguous share [lo, hi) of n items
+void shard_bounds(int64_t n, int rank, int world, int64_t* lo, int64_t* hi) {
+  const int64_t per = (n + world - 1) / world;
+  *lo = std::min(n, (int64_t)rank * per);
+  *hi = std::min(n, *lo + per);
+}
 
 }  // namespace
 
@@ -481,14 +502,23 @@ AHV_API size_t ahv_peer_bytes(int max_pairs, int max_k) {
   return (max_pairs < 1 || !k_ok(max_k)) ? 0 : peer::buffer_bytes(max_pairs, max_k);
 }
 
-AHV_API int ahv_peer_alloc(int max_pairs, int max_k, void** ptr) {
-  if (!ptr || max_pairs < 1 || !k_ok(max_k)) return AHV_EINVAL;
+AHV_API size_t ahv_peer_bytes_ex(int max_pairs, int max_k, int64_t max_hyps) {
+  return (max_pairs < 1 || !k_ok(max_k) || !n_ok(max_hyps)) ? 0 : peer::buffer_bytes_ex(max_pairs, max_k, max_hyps);
+}
+
+AHV_API int ahv_peer_alloc_ex(int max_pairs, int max_k, int64_t max_hyps, void** ptr) {
+  if (!ptr || max_pairs < 1 || !k_ok(max_k) || !n_ok(max_hyps)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
-  const size_t bytes = peer::buffer_bytes(max_pairs, max_k);
+  st = preload_exchange_kernels();
+  if (st != AHV_OK) return st;
+  const size_t bytes = peer::buffer_bytes_ex(max_pairs, max_k, max_hyps);
   if (cudaMalloc(ptr, bytes) != cudaSuccess) return AHV_ECUDA;
-  const uint32_t hdr[4] = {0u, 0u, (uint32_t)max_pairs, (uint32_t)max_k};  // seq, err, capacity
+  const uint32_t hdr[4] = {0u, 0u, (uint32_t)max_pairs, (uint32_t)max_k};  // seq, err, capacity (cap_hyps below)
+  const uint32_t cap_hyps = (uint32_t)max_hyps;
   if (cudaMemset(*ptr, 0, bytes) != cudaSuccess || cudaMemcpy(*ptr, hdr, sizeof(hdr), cudaMemcpyHostToDevice) != cudaSuccess ||
+      cudaMemcpy(static_cast<uint32_t*>(*ptr) + peer::kHdrCapHyps, &cap_hyps, sizeof(cap_hyps), cudaMemcpyHostToDevice) !=
+          cudaSuccess ||
       cudaDeviceSynchronize() != cudaSuccess) {
     cudaFree(*ptr);
     *ptr = nullptr;
@@ -496,6 +526,8 @@ AHV_API int ahv_peer_alloc(int max_pairs, int max_k, void** ptr) {
   }
   return AHV_OK;
 }
+
+AHV_API int ahv_peer_alloc(int max_pairs, int max_k, void** ptr) { return ahv_peer_alloc_ex(max_pairs, max_k, 0, ptr); }
 
 AHV_API int ahv_peer_free(void* ptr) { return (!ptr || cudaFree(ptr) == cudaSuccess) ? AHV_OK : AHV_ECUDA; }
 
@@ -531,6 +563,16 @@ AHV_API int ahv_peer_capacity(const void* buf, int* max_pairs, int* max_k) {
   if (cudaMemcpy(hdr, buf, sizeof(hdr), cudaMemcpyDeviceToHost) != cudaSuccess) return AHV_ECUDA;  // synchronises
   *max_pairs = (int)hdr[2];
   *max_k = (int)hdr[3];
+  return AHV_OK;
+}
+
+AHV_API int ahv_peer_capacity_ex(const void* buf, int* max_pairs, int* max_k, int64_t* max_hyps) {
+  if (!buf || !max_pairs || !max_k || !max_hyps) return AHV_EINVAL;
+  unsigned hdr[5];
+  if (cudaMemcpy(hdr, buf, sizeof(hdr), cudaMemcpyDeviceToHost) != cudaSuccess) return AHV_ECUDA;  // synchronises
+  *max_pairs = (int)hdr[2];
+  *max_k = (int)hdr[3];
+  *max_hyps = (int64_t)hdr[peer::kHdrCapHyps];
   return AHV_OK;
 }
 
@@ -626,6 +668,99 @@ AHV_API int ahv_verify_sharded(const void* vol_src, int vol_dtype, const float* 
     if (st != AHV_OK) return st;
   }
   return launch_topk_exchange(l_val, l_idx, R, r_per_pair != 0, idx_offset, N, B, k, topk_val, topk_idx, R_best, pa, s);
+}
+
+AHV_API int ahv_scores_exchange(const float* part, int B, int64_t N, float* scores, int rank, int world, void* const* peers,
+                                int peer_max_pairs, int peer_max_k, int64_t peer_max_hyps, void* stream) {
+  if (B < 1 || N < 1 || !n_ok(N) || !scores) return AHV_EINVAL;
+  peer::Args pa;
+  int st = make_peer_args(rank, world, peers, peer_max_pairs, peer_max_k, &pa);
+  if (st != AHV_OK) return st;
+  if (world < 2 || B > peer_max_pairs || !n_ok(peer_max_hyps) || N > peer_max_hyps) return AHV_EINVAL;
+  int64_t lo, hi;
+  shard_bounds(N, rank, world, &lo, &hi);
+  if (hi > lo && !part) return AHV_EINVAL;
+  st = check_device();
+  if (st != AHV_OK) return st;
+  return launch_scores_exchange(part, B, N, scores, pa, peer_max_hyps, (cudaStream_t)stream);
+}
+
+AHV_API size_t ahv_refine_gradient_sharded_workspace_bytes(int B, int64_t N, int k, int world) {
+  if (B < 0 || N < 0 || !k_ok(k) || world < 1 || world > peer::kMaxPeers) return 0;
+  return world == 1 ? RefineGradientWs(B, N, k).total : ShardedRefineWs(B, N, k, world).total;
+}
+
+AHV_API int ahv_refine_gradient_sharded(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R,
+                                        int r_per_pair, const float* W1, const float* W2, const float* b2, const float* base,
+                                        int k, int steps, float step_deg, float min_sep_deg, float* first_val,
+                                        int64_t* first_idx, float* first_R, float* R_all, float* score_all, float* best_val,
+                                        int64_t* best_idx, float* R_best, int B, int64_t N, int math_mode, void* workspace,
+                                        size_t workspace_bytes, int rank, int world, void* const* peers, int peer_max_pairs,
+                                        int peer_max_k, int64_t peer_max_hyps, void* stream) {
+  if (B < 1 || N < 1 || !n_ok(N) || !k_ok(k) || k > N) return AHV_EINVAL;
+  if (!ascent_args_ok(vol_dtype, steps, step_deg) || !min_sep_ok(min_sep_deg) || !math_mode_ok(math_mode)) return AHV_EINVAL;
+  if (!all_set(vol_src, vol_tgt, R, W1, W2, b2, base, first_val, first_idx, first_R, R_all, score_all, best_val, best_idx,
+               workspace))
+    return AHV_EINVAL;
+  if (!all_aligned16(vol_src, vol_tgt, R, W1, W2, first_R, R_all, R_best, workspace)) return AHV_EINVAL;
+  peer::Args pa;
+  int st = make_peer_args(rank, world, peers, peer_max_pairs, peer_max_k, &pa);
+  if (st != AHV_OK) return st;
+  const bool distinct = min_sep_deg > 0.0f;
+  if (world > 1 && (B > peer_max_pairs || k > peer_max_k)) return AHV_EINVAL;  // the slot gather's entries
+  if (world > 1 && distinct && (!n_ok(peer_max_hyps) || N > peer_max_hyps)) return AHV_EINVAL;  // the score region
+  if (world == 1)
+    return refine_gradient(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, min_sep_deg,
+                           first_val, first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode,
+                           workspace, workspace_bytes, stream);
+  const ShardedRefineWs w(B, N, k, world);
+  if (workspace_bytes < w.total) return AHV_EWORKSPACE;
+  st = check_device();
+  if (st != AHV_OK) return st;
+  cudaStream_t s = (cudaStream_t)stream;
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  float* rs = reinterpret_cast<float*>(ws + w.rs);
+  float* tgt = reinterpret_cast<float*>(ws + w.tgt);
+  int64_t lo, hi;
+  shard_bounds(N, rank, world, &lo, &hi);
+  const int64_t n = hi - lo;
+  if (n > 0)  // this rank's rotations, 16-byte aligned for the scorers (a shared set: one row)
+    AHV_CUDA_OK(cudaMemcpy2DAsync(rs, (size_t)n * 9 * sizeof(float), R + (size_t)lo * 9, (size_t)N * 9 * sizeof(float),
+                                  (size_t)n * 9 * sizeof(float), r_per_pair ? B : 1, cudaMemcpyDeviceToDevice, s));
+  if (!distinct) {
+    // pass 1: the slice's top-k, exchanged and merged into the whole set's top-k with its rotations
+    st = ahv_verify_sharded(vol_src, vol_dtype, vol_tgt, rs, r_per_pair, W1, W2, b2, base, first_val, first_idx, first_R, k, lo,
+                            B, n, math_mode, ws, w.rs, rank, world, peers, peer_max_pairs, peer_max_k, stream);
+    if (st != AHV_OK) return st;
+  }
+  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
+  if (st != AHV_OK) return st;
+  if (distinct) {
+    // pass 1: the slice's scores, all-gathered into the whole [B,N] on every rank, then the SAME greedy selection
+    // over the whole set on every rank (per-shard NMS lists do not merge into the global one)
+    float* full = reinterpret_cast<float*>(ws + w.full);
+    if (n > 0) {
+      st = ahv_score(vol_src, vol_dtype, tgt, rs, r_per_pair, W1, W2, b2, base, nullptr, nullptr, nullptr, 0, 0, B, n,
+                     math_mode, ws, w.rs, stream);
+      if (st != AHV_OK) return st;
+    }
+    st = launch_scores_exchange(reinterpret_cast<const float*>(ws), B, N, full, pa, peer_max_hyps, s);
+    if (st != AHV_OK) return st;
+    st = launch_topk_distinct(full, R, r_per_pair != 0, B, N, k, min_sep_deg, first_val, first_idx, first_R, s);
+    if (st != AHV_OK) return st;
+  }
+  // this rank's share of the B*k ascents, then every ascended slot to every rank
+  int64_t ilo, ihi;
+  shard_bounds((int64_t)B * k, rank, world, &ilo, &ihi);
+  st = launch_gradient_ascent(vol_src, vol_dtype, tgt, first_R, W1, W2, b2, base, steps, step_deg, R_all, score_all, B, k, s,
+                              distinct ? first_idx : nullptr, ilo, ihi);
+  if (st != AHV_OK) return st;
+  st = launch_slot_gather(R_all, score_all, ilo, ihi, B, k, pa, s);
+  if (st != AHV_OK) return st;
+  // per-pair arg-max over the k ascended candidates, on every rank
+  st = launch_topk(score_all, B, k, 1, 0, best_val, best_idx, ws + w.top, w.total - w.top, s);
+  if (st != AHV_OK || !R_best) return st;
+  return launch_gather_rotations(R_all, 1, best_idx, 0, B, k, 1, R_best, s);
 }
 
 // ---- host-buffer entries -------------------------------------------------------------------------------

@@ -67,17 +67,21 @@ __device__ __forceinline__ void trial_rotation(const float* R, const float* G, f
     }
 }
 
-template <typename T>
+// kItemRange: the grid covers items [item_lo, item_hi) of the B*K only (one rank's share in
+// ahv_refine_gradient_sharded); without it the range is [0, B*K) and the arguments are unused.
+template <typename T, bool kItemRange>
 __global__ void __launch_bounds__(kThreads, 1)
 ascent_fp32_kernel(const T* __restrict__ vol_src, const float* __restrict__ tgt_feat, const float* __restrict__ R_init,
                    const float* __restrict__ W1, const float* __restrict__ W2, const float* __restrict__ b2,
                    const float* __restrict__ base, int steps, float theta0, float* __restrict__ R_out,
-                   float* __restrict__ score_out, int B, int K, const int64_t* __restrict__ skip_idx) {
+                   float* __restrict__ score_out, int B, int K, const int64_t* __restrict__ skip_idx,
+                   int64_t item_lo, int64_t item_hi) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   AscentSmem& as = *reinterpret_cast<AscentSmem*>(smem_raw);
   Fp32Smem& sm = as.f;
-  const int64_t total = (int64_t)B * K;
-  const int64_t lo = total * blockIdx.x / gridDim.x, hi = total * (blockIdx.x + 1) / gridDim.x;
+  const int64_t first = kItemRange ? item_lo : 0;
+  const int64_t total = kItemRange ? item_hi - item_lo : (int64_t)B * K;
+  const int64_t lo = first + total * blockIdx.x / gridDim.x, hi = first + total * (blockIdx.x + 1) / gridDim.x;
   if (lo >= hi) return;
   const int t = threadIdx.x;
   stage_weights(sm, W1, W2, base);
@@ -147,27 +151,56 @@ ascent_fp32_kernel(const T* __restrict__ vol_src, const float* __restrict__ tgt_
   }
 }
 
+template <bool kItemRange>
+void launch_ascent(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R_init, const float* W1,
+                   const float* W2, const float* b2, const float* base, int steps, float theta0, float* R_out,
+                   float* score_out, int B, int K, const int64_t* skip_idx, int64_t item_lo, int64_t item_hi,
+                   unsigned grid, size_t smem, cudaStream_t s, cudaError_t* err) {
+  if (vol_dtype == AHV_VOL_F32) {
+    *err = cudaFuncSetAttribute(ascent_fp32_kernel<float, kItemRange>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (*err != cudaSuccess) return;
+    ascent_fp32_kernel<float, kItemRange><<<grid, kThreads, smem, s>>>((const float*)vol_src, tgt_feat, R_init, W1, W2, b2,
+                                                                       base, steps, theta0, R_out, score_out, B, K, skip_idx,
+                                                                       item_lo, item_hi);
+  } else {
+    *err = cudaFuncSetAttribute(ascent_fp32_kernel<__nv_bfloat16, kItemRange>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)smem);
+    if (*err != cudaSuccess) return;
+    ascent_fp32_kernel<__nv_bfloat16, kItemRange><<<grid, kThreads, smem, s>>>((const __nv_bfloat16*)vol_src, tgt_feat, R_init,
+                                                                               W1, W2, b2, base, steps, theta0, R_out,
+                                                                               score_out, B, K, skip_idx, item_lo, item_hi);
+  }
+  *err = cudaGetLastError();
+}
+
 int launch_gradient_ascent(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R_init, const float* W1,
                            const float* W2, const float* b2, const float* base, int steps, float step_deg, float* R_out,
-                           float* score_out, int B, int K, cudaStream_t s, const int64_t* skip_idx) {
-  const int64_t total = (int64_t)B * K;
-  if (total == 0) return AHV_OK;
+                           float* score_out, int B, int K, cudaStream_t s, const int64_t* skip_idx, int64_t item_lo,
+                           int64_t item_hi) {
+  const bool ranged = item_hi >= 0;
+  const int64_t total = ranged ? item_hi - item_lo : (int64_t)B * K;
+  if (total <= 0) return AHV_OK;
   int dev = 0, sms = 0;
   AHV_CUDA_OK(cudaGetDevice(&dev));
   AHV_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   const unsigned grid = (unsigned)(total < sms ? total : sms);
   const size_t smem = sizeof(AscentSmem);
   const float theta0 = (float)((double)step_deg * (3.14159265358979323846 / 180.0));  // math.radians, rounded once
-  if (vol_dtype == AHV_VOL_F32) {
-    AHV_CUDA_OK(cudaFuncSetAttribute(ascent_fp32_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ascent_fp32_kernel<float><<<grid, kThreads, smem, s>>>((const float*)vol_src, tgt_feat, R_init, W1, W2, b2, base, steps,
-                                                           theta0, R_out, score_out, B, K, skip_idx);
-  } else {
-    AHV_CUDA_OK(cudaFuncSetAttribute(ascent_fp32_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ascent_fp32_kernel<__nv_bfloat16><<<grid, kThreads, smem, s>>>((const __nv_bfloat16*)vol_src, tgt_feat, R_init, W1, W2,
-                                                                   b2, base, steps, theta0, R_out, score_out, B, K, skip_idx);
-  }
-  AHV_CUDA_OK(cudaGetLastError());
+  cudaError_t err = cudaSuccess;
+  if (ranged)
+    launch_ascent<true>(vol_src, vol_dtype, tgt_feat, R_init, W1, W2, b2, base, steps, theta0, R_out, score_out, B, K, skip_idx,
+                        item_lo, item_hi, grid, smem, s, &err);
+  else
+    launch_ascent<false>(vol_src, vol_dtype, tgt_feat, R_init, W1, W2, b2, base, steps, theta0, R_out, score_out, B, K, skip_idx,
+                         0, 0, grid, smem, s, &err);
+  AHV_CUDA_OK(err);
+  return AHV_OK;
+}
+
+int preload_ranged_ascent() {
+  cudaFuncAttributes a;
+  AHV_CUDA_OK(cudaFuncGetAttributes(&a, ascent_fp32_kernel<float, true>));
+  AHV_CUDA_OK(cudaFuncGetAttributes(&a, ascent_fp32_kernel<__nv_bfloat16, true>));
   return AHV_OK;
 }
 

@@ -217,7 +217,8 @@ int launch_infonce(const float* scores, const float* R, int r_per_pair, const fl
                    float* loss, float* grad, int B, int64_t N, cudaStream_t s);
 int launch_gradient_ascent(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R_init, const float* W1,
                            const float* W2, const float* b2, const float* base, int steps, float step_deg, float* R_out,
-                           float* score_out, int B, int K, cudaStream_t s, const int64_t* skip_idx = nullptr);
+                           float* score_out, int B, int K, cudaStream_t s, const int64_t* skip_idx = nullptr,
+                           int64_t item_lo = 0, int64_t item_hi = -1);  // item_hi < 0: every item of B*K
 int launch_forward_3d2d(const float* vol, const float* W1, const float* W2, const float* b2,
                         float* feat, int64_t m, cudaStream_t s);
 int launch_tgt_feat(const float* vol_tgt, const float* W1, const float* W2, const float* b2,
@@ -239,6 +240,12 @@ int launch_verify_tc_argmax(const void* vol_src, int vol_dtype, const float* vol
 int launch_topk_exchange(const float* val, const int64_t* idx, const float* R, int r_per_pair, int64_t idx_offset,
                          int64_t N, int B, int k, float* out_val, int64_t* out_idx, float* R_best,
                          const peer::Args& pa, cudaStream_t s);
+int launch_scores_exchange(const float* part, int B, int64_t N, float* out, const peer::Args& pa, int64_t cap_hyps,
+                           cudaStream_t s);
+int launch_slot_gather(float* R_all, float* score_all, int64_t item_lo, int64_t item_hi, int B, int k, const peer::Args& pa,
+                       cudaStream_t s);
+int preload_exchange_kernels();  // see ahv_exchange.cu
+int preload_ranged_ascent();
 int launch_topk(const float* scores, int B, int64_t N, int k, int64_t idx_offset, float* val,
                 int64_t* idx, void* ws, size_t ws_bytes, cudaStream_t s);
 size_t topk_workspace_bytes(int B, int64_t N, int k);

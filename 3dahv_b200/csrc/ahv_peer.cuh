@@ -7,6 +7,18 @@
 // exchanges of different sizes may follow one another.  Exchange s uses parity s & 1.  A rank can only finish
 // exchange s+1 after every peer has sent s+1, i.e. after every peer is done reading exchange s, so two parities
 // suffice; sequence numbers make the flags self-cleaning (CUDA-graph replay needs no host-side reset).
+//
+// Optional score region (ahv_peer_alloc_ex with max_hyps > 0; cap_hyps is header word 4, 0 = none):
+//   [entries end, ...)  scores[2 parity][cap_pairs][cap_hyps] fp32: exchange s of ahv_scores_exchange leaves the
+//                       whole [B,N] matrix in every rank's parity s & 1 plane (each rank stores its columns [lo,hi))
+// Header words 5 and 6 are private to the owning rank: the CTA ticket of a scores exchange (back to 0 when the
+// exchange ends) and that exchange's outcome (0 = complete, 1 = a peer never arrived), read by the copy-out.
+// The stride again depends on the capacity only.  Two parities suffice here as well, because the matrix is read
+// out of the region by a SECOND, stream-ordered launch (score_copyout_kernel) that precedes the rank's next
+// exchanging launch: rank q announces exchange s+1 only after it has copied exchange s out, so a peer that sees
+// q's flag s+1 (which it must before it completes s+1 and starts s+2, the next user of the plane) can no longer
+// overwrite anything q has still to read.  A caller that inserted another exchanging launch between the two would
+// break this; the entry points never do.
 #pragma once
 #include "ahv_common.cuh"
 
@@ -27,6 +39,13 @@ __host__ __device__ inline size_t entry_off(int par, int r, int cap_pairs, int c
   return (size_t)kEntriesOff + ((((size_t)par * kMaxPeers + r) * cap_pairs + b) * cap_k + j) * kEntryBytes;
 }
 __host__ inline size_t buffer_bytes(int cap_pairs, int cap_k) { return entry_off(2, 0, cap_pairs, cap_k, 0, 0); }
+constexpr int kHdrCapHyps = 4, kHdrTicket = 5, kHdrScoresStatus = 6;  // uint32 header words of the score region
+__host__ __device__ inline size_t score_off(int par, int cap_pairs, int cap_k, int64_t cap_hyps, int b, int64_t n) {
+  return entry_off(2, 0, cap_pairs, cap_k, 0, 0) + (((size_t)par * cap_pairs + b) * (size_t)cap_hyps + (size_t)n) * sizeof(float);
+}
+__host__ inline size_t buffer_bytes_ex(int cap_pairs, int cap_k, int64_t cap_hyps) {
+  return score_off(2, cap_pairs, cap_k, cap_hyps, 0, 0);
+}
 
 __device__ __forceinline__ uint32_t ordered_bits(float score) {  // same order as make_key()
   uint32_t u = __float_as_uint(score + 0.0f);

@@ -49,9 +49,11 @@ class PeerExchange:
     (`ahv_peer_alloc`), sends its CUDA IPC handle to the peers (one all-gather of 64 bytes at set-up) and maps
     theirs, after which the scoring kernels talk to each other through NVLink peer memory and a verification
     step involves no NCCL call at all.  One instance per process group; it serves any call with B <= max_pairs and
-    k <= max_k (the entry stride depends on the capacity only, so B and k may change from step to step)."""
+    k <= max_k (the entry stride depends on the capacity only, so B and k may change from step to step).
+    max_hyps > 0 adds a score region (`ahv_peer_alloc_ex`, 2 * max_pairs * max_hyps * 4 bytes) through which
+    `ShardedVerifier.scores` and the distinct selection all-gather [B,N] score matrices with N <= max_hyps."""
 
-    def __init__(self, max_pairs: int, device, group=None, max_k: int = 1):
+    def __init__(self, max_pairs: int, device, group=None, max_k: int = 1, max_hyps: int = 0):
         import ctypes
 
         from . import _lib
@@ -62,7 +64,9 @@ class PeerExchange:
             raise ValueError("the peer exchange covers the GPUs of one node (<= 8)")
         if not (1 <= max_k <= 32) or max_pairs < 1:
             raise ValueError("max_pairs >= 1 and 1 <= max_k <= 32 expected")
-        self.max_pairs, self.max_k = max_pairs, max_k
+        if not 0 <= max_hyps < 2**31:
+            raise ValueError("0 <= max_hyps < 2**31 expected")
+        self.max_pairs, self.max_k, self.max_hyps = max_pairs, max_k, max_hyps
         self.device = torch.device(device)
         lib = _lib.lib()
         self._lib = lib
@@ -74,7 +78,7 @@ class PeerExchange:
         own = ctypes.c_void_p()
         handle = ctypes.create_string_buffer(64)
         with torch.cuda.device(self.device):
-            if lib.ahv_peer_alloc(max_pairs, max_k, ctypes.byref(own)) != 0:
+            if lib.ahv_peer_alloc_ex(max_pairs, max_k, max_hyps, ctypes.byref(own)) != 0:
                 ok = False
             elif lib.ahv_peer_export(own, handle) != 0:
                 ok = False
@@ -155,12 +159,23 @@ class ShardedVerifier:
         r = self.verifier.score(vol_src, vol_tgt, R_slice, k=k, return_scores=False, idx_offset=idx_offset, gather=False)
         return r.topk_val, r.topk_idx
 
+    def _stepped(self):
+        """Counts a peer-exchanging call; every `check_every` of them, raises if one timed out."""
+        self._steps += 1
+        if self.check_every and self._steps % self.check_every == 0:
+            self.peer.check()
+
     @torch.no_grad()
-    def score(self, vol_src, vol_tgt, R, k: int = 1):
-        """Returns (topk_val [B,k], topk_idx [B,k] global, R_best [B,k,3,3])."""
+    def score(self, vol_src, vol_tgt, R, k: int = 1, min_sep_deg: float = 0.0):
+        """Returns (topk_val [B,k], topk_idx [B,k] global, R_best [B,k,3,3]).  min_sep_deg > 0: the k best rotations
+        pairwise more than min_sep_deg apart, as `HypothesisVerifier.score(min_sep_deg=...)` gives them on one GPU.
+        Greedy suppression does not compose from per-shard lists, so the whole [B,N] matrix is assembled on every rank
+        (`scores`) and `ops.topk_distinct` runs on every rank over the whole set."""
         per_pair = R.dim() == 4
         N = R.shape[1] if per_pair else R.shape[0]
         k = min(k, N)
+        if min_sep_deg > 0:
+            return ops.topk_distinct(self.scores(vol_src, vol_tgt, R), R, k, min_sep_deg)
         lo, hi = shard_bounds(N, self.rank, self.world)
         B = vol_src.shape[0]
         if (self.peer is not None and self.world > 1 and B <= self.peer.max_pairs and k <= self.peer.max_k
@@ -173,9 +188,7 @@ class ShardedVerifier:
             vs = vol_src if vol_src.dtype == torch.bfloat16 else vol_src.float()
             val, idx, Rb = ops.verify_sharded(vs, vol_tgt.float(), Rs, W1, W2, b2, lo, self.peer, k=k, math=v.math,
                                               workspace=v._workspace(B, hi - lo, k, vol_src.device))
-            self._steps += 1
-            if self.check_every and self._steps % self.check_every == 0:
-                self.peer.check()
+            self._stepped()
             return val, idx, Rb
         if hi > lo:
             Rs = (R[:, lo:hi] if per_pair else R[lo:hi]).contiguous()
@@ -213,19 +226,79 @@ class ShardedVerifier:
         return R_best[:, 0], val[:, 0], (first_val, first_idx, first_R), cand
 
     @torch.no_grad()
+    def refine_by_gradient(self, vol_src, vol_tgt, R, k: int = 32, steps: int = 20, step_deg: float = 1.0,
+                           min_sep_deg: float = 0.0):
+        """`HypothesisVerifier.refine_by_gradient` over a sharded set (BASELINE config 4's accurate path on several
+        GPUs): every rank passes the WHOLE set and gets the one-GPU result bit for bit.  The grid pass is sharded;
+        with min_sep_deg > 0 the distinct selection runs on every rank over the assembled score matrix; each rank
+        ascends its share of the B*k (pair, slot) items and the ascended slots are gathered.  With a `peer` exchange
+        (max_hyps >= N for min_sep_deg > 0) the whole chain is one C call with no NCCL call
+        (`ops.refine_gradient_sharded`); without, it is composed of NCCL all-gathers and the one-GPU ops.
+        Returns (R_best [B,3,3], score [B], first pass as a VerifyResult, R_all [B,k,3,3], score_all [B,k])."""
+        from .verify import VerifyResult, _src_volume
+
+        v = self.verifier
+        per_pair = R.dim() == 4
+        N = R.shape[1] if per_pair else R.shape[0]
+        k = min(k, N)
+        B = vol_src.shape[0]
+        if self.world == 1:
+            return v.refine_by_gradient(vol_src, vol_tgt, R, k=k, steps=steps, step_deg=step_deg, min_sep_deg=min_sep_deg)
+        dev = vol_src.device
+        W1, W2, b2 = v._weights_on(dev)
+        p = self.peer
+        if (p is not None and B <= p.max_pairs and k <= p.max_k and (min_sep_deg == 0 or N <= p.max_hyps)):
+            fv, fi, fR, Ra, sa, bv, bi, bR, self._ws_refine_gradient = ops.refine_gradient_sharded(
+                _src_volume(vol_src), vol_tgt.float(), R, W1, W2, b2, p, k=k, steps=steps, step_deg=step_deg, math=v.math,
+                workspace=getattr(self, "_ws_refine_gradient", None), min_sep_deg=min_sep_deg)
+            self._stepped()
+            return bR, bv, VerifyResult(None, fv, fi, fR), Ra, sa
+        # NCCL composition: first pass over the whole set, this rank's share of the ascents, all-gather of the slots
+        fv, fi, fR = self.score(vol_src, vol_tgt, R, k=k, min_sep_deg=min_sep_deg)
+        total = B * k
+        ilo, ihi = shard_bounds(total, self.rank, self.world)
+        per = -(-total // self.world)
+        R_part = torch.zeros(per, 9, device=dev, dtype=torch.float32)
+        s_part = torch.zeros(per, device=dev, dtype=torch.float32)
+        if ihi > ilo:
+            pair = torch.arange(ilo, ihi, device=dev) // k
+            tgt = v.target_features(vol_tgt)[pair]
+            Ri, si = ops.gradient_ascent(_src_volume(vol_src)[pair], tgt, fR.reshape(total, 1, 3, 3)[ilo:ihi], W1, W2, b2,
+                                         steps=steps, step_deg=step_deg)
+            empty = fi.reshape(total)[ilo:ihi] < 0        # empty distinct slots are not ascended
+            R_part[:ihi - ilo] = torch.where(empty[:, None], torch.full_like(Ri.reshape(-1, 9), float("nan")), Ri.reshape(-1, 9))
+            s_part[:ihi - ilo] = torch.where(empty, torch.full_like(si.reshape(-1), float("-inf")), si.reshape(-1))
+        Rs = [torch.empty_like(R_part) for _ in range(self.world)]
+        ss = [torch.empty_like(s_part) for _ in range(self.world)]
+        dist.all_gather(Rs, R_part, group=self.group)
+        dist.all_gather(ss, s_part, group=self.group)
+        R_all = torch.cat(Rs)[:total].reshape(B, k, 3, 3).contiguous()
+        s_all = torch.cat(ss)[:total].reshape(B, k).contiguous()
+        val, idx = ops.topk(s_all, 1)
+        return ops.gather_rotations(R_all, idx)[:, 0], val[:, 0], VerifyResult(None, fv, fi, fR), R_all, s_all
+
+    @torch.no_grad()
     def scores(self, vol_src, vol_tgt, R):
         """The full pred_sim [B,N] (modules/model.py:193) of a sharded set on every rank: each rank scores its slice,
-        one NCCL all-gather of B*N/P floats per rank puts the matrix together (SURVEY.md §8e; 25.6 MB per rank at
-        B=128, N=50 000, P=8).  Only needed when the caller wants every score; selection never moves them."""
+        and the slices are all-gathered - through the score region of `peer` (NVLink, no NCCL call) when it has
+        max_hyps >= N and max_pairs >= B, else with one NCCL all-gather of B*N/P floats per rank (SURVEY.md §8e;
+        25.6 MB per rank at B=128, N=50 000, P=8).  Only needed when the caller wants every score, or for the
+        distinct selection; the plain top-k never moves them."""
         per_pair = R.dim() == 4
         N = R.shape[1] if per_pair else R.shape[0]
         B = vol_src.shape[0]
         per = -(-N // self.world)
         lo, hi = shard_bounds(N, self.rank, self.world)
-        part = torch.zeros(B, per, device=vol_src.device, dtype=torch.float32)     # equal-sized pieces for the all-gather
+        p = self.peer
+        via_peer = p is not None and self.world > 1 and N <= getattr(p, "max_hyps", 0) and B <= p.max_pairs
+        part = torch.zeros(B, hi - lo if via_peer else per, device=vol_src.device, dtype=torch.float32)
         if hi > lo:
             Rs = (R[:, lo:hi] if per_pair else R[lo:hi]).contiguous()
             part[:, :hi - lo] = self.verifier.score(vol_src, vol_tgt, Rs, k=1, return_scores=True).scores
+        if via_peer:
+            out = ops.scores_exchange(part, N, p)
+            self._stepped()
+            return out
         if self.world == 1:
             return part[:, :N]
         pieces = [torch.empty_like(part) for _ in range(self.world)]

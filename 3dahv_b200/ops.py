@@ -516,6 +516,64 @@ def topk_exchange(val, idx, R, idx_offset: int, peer):
     return out_v, out_i, Rb
 
 
+def scores_exchange(part, N: int, peer, out=None):
+    """ahv_scores_exchange: this rank's columns part [B, hi-lo] (lo, hi = `dist.shard_bounds(N, rank, world)`) of a
+    [B,N] score matrix -> the whole [B,N] on every rank, through the score region of `peer` (a `dist.PeerExchange`
+    with max_hyps >= N).  `out`: a [B,N] fp32 tensor to write into (CUDA-graph replays)."""
+    from .dist import shard_bounds
+
+    p = _dev(part, "part")
+    B = p.shape[0]
+    lo, hi = shard_bounds(N, peer.rank, peer.world)
+    if p.dim() != 2 or p.shape[1] != hi - lo:
+        raise ValueError(f"part must be [B,{hi - lo}] (rank {peer.rank}'s columns [{lo},{hi}) of N={N})")
+    max_hyps = getattr(peer, "max_hyps", 0)
+    if B > peer.max_pairs or N > max_hyps:
+        raise ValueError(f"exchange buffer holds {peer.max_pairs} pairs x {max_hyps} scores; got B={B}, N={N}")
+    out = torch.empty(B, N, device=p.device, dtype=torch.float32) if out is None else out
+    _call("ahv_scores_exchange", p.device, p.data_ptr() if hi > lo else None, B, N, out.data_ptr(), peer.rank, peer.world,
+          _peer_array(peer), peer.max_pairs, peer.max_k, max_hyps)
+    return out
+
+
+def refine_gradient_sharded(vol_src, vol_tgt, R, W1, W2, b2, peer, k: int = 32, steps: int = 20, step_deg: float = 1.0,
+                            math: int = MATH_TC, workspace: torch.Tensor | None = None, out=None, min_sep_deg: float = 0.0):
+    """ahv_refine_gradient_sharded: `refine_gradient` over a rotation set sharded across the ranks of `peer` (a
+    `dist.PeerExchange`).  Every rank passes the WHOLE set R and gets the whole-set result, bit for bit what
+    `refine_gradient` returns on one GPU: the rank scores its `dist.shard_bounds` slice, the kernels exchange the
+    first pass (top-k lists, or with min_sep_deg > 0 the score matrix, after which the distinct selection runs on
+    every rank) and the ascended slots through NVLink peer memory.  min_sep_deg > 0 needs peer.max_hyps >= N.
+    One C call, no NCCL, CUDA-graph capturable (`out` = a previous result's tuple).  Returns `refine_gradient`'s tuple."""
+    vs, vdt = _vol_src(vol_src)
+    vt = _dev(vol_tgt, "vol_tgt")
+    B = vs.shape[0]
+    R, per_pair, N = _rotations(_dev(R, "R"), B)
+    if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
+        raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
+    if not 1 <= k <= min(32, N):
+        raise ValueError("1 <= k <= min(32, N) expected")
+    max_hyps = getattr(peer, "max_hyps", 0)
+    if peer.world > 1 and (B > peer.max_pairs or k > peer.max_k or (min_sep_deg > 0 and N > max_hyps)):
+        raise ValueError(f"exchange buffer holds {peer.max_pairs} pairs x top-{peer.max_k} x {max_hyps} scores; got B={B}, k={k}, "
+                         f"N={N}")
+    W1, W2, b2 = _head(W1, W2, b2)
+    dev = vs.device
+    if out is None:
+        f = dict(device=dev, dtype=torch.float32)
+        out = (torch.empty(B, k, **f), torch.empty(B, k, device=dev, dtype=torch.int64), torch.empty(B, k, 3, 3, **f),
+               torch.empty(B, k, 3, 3, **f), torch.empty(B, k, **f), torch.empty(B, **f),
+               torch.empty(B, device=dev, dtype=torch.int64), torch.empty(B, 3, 3, **f))
+    fv, fi, fR, Ra, sa, bv, bi, bR = out[:8]
+    need = int(_lib.lib().ahv_refine_gradient_sharded_workspace_bytes(B, N, k, peer.world))
+    workspace, ws_bytes = _workspace(workspace, need, dev)
+    _call("ahv_refine_gradient_sharded", dev, vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(),
+          W2.data_ptr(), b2.data_ptr(), base_coords(dev).data_ptr(), k, int(steps), float(step_deg), float(min_sep_deg),
+          fv.data_ptr(), fi.data_ptr(), fR.data_ptr(), Ra.data_ptr(), sa.data_ptr(), bv.data_ptr(), bi.data_ptr(), bR.data_ptr(),
+          B, N, math, workspace.data_ptr(), ws_bytes, peer.rank, peer.world, _peer_array(peer), peer.max_pairs, peer.max_k,
+          max_hyps)
+    return fv, fi, fR, Ra, sa, bv, bi, bR, workspace
+
+
 def topk(scores: torch.Tensor, k: int, idx_offset: int = 0):
     """torch.max / top-k with the reference's tie rule (lowest index wins)."""
     s = _dev(scores, "scores")

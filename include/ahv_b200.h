@@ -368,6 +368,51 @@ AHV_API int ahv_verify_sharded(const void* vol_src, int vol_dtype, const float* 
                                int math_mode, void* workspace, size_t workspace_bytes, int rank, int world,
                                void* const* peers, int peer_max_pairs, int peer_max_k, void* stream);
 
+/* Exchange buffers with a score region (extension): ahv_peer_alloc_ex(max_pairs, max_k, max_hyps) adds
+ * 2 x max_pairs x max_hyps fp32 after the entries, for ahv_scores_exchange of up to max_pairs x max_hyps scores;
+ * max_hyps == 0 is ahv_peer_alloc (same size, same layout), 0 <= max_hyps <= 2^31 - 1.  ahv_peer_bytes_ex gives the
+ * size (0 for invalid capacities), ahv_peer_capacity_ex reads all three capacities back (synchronising).  A buffer
+ * of either kind serves every other exchanging entry, with the same sequence counter. */
+AHV_API size_t ahv_peer_bytes_ex(int max_pairs, int max_k, int64_t max_hyps);
+AHV_API int ahv_peer_alloc_ex(int max_pairs, int max_k, int64_t max_hyps, void** ptr);
+AHV_API int ahv_peer_capacity_ex(const void* buf, int* max_pairs, int* max_k, int64_t* max_hyps);
+
+/* All-gather of a score matrix sliced by hypothesis, through the score region (extension): part [B, hi-lo] fp32 =
+ * columns [lo, hi) of [B,N], where lo = min(N, rank*ceil(N/world)) and hi = min(N, lo + ceil(N/world)) (the
+ * partition of dist.shard_bounds; part may be NULL when the slice is empty); scores [B,N] receives the whole matrix,
+ * the same on every rank.  B <= peer_max_pairs, 1 <= N <= peer_max_hyps (the buffers' ahv_peer_alloc_ex capacity),
+ * world >= 2.  Two launches: a grid that stores the slice into every rank's region, whose last CTA alone announces
+ * the exchange and waits for the peers, then a copy into `scores`.  A peer that never arrives gives NaN scores after
+ * ~20 s, as for the other exchanges.  No host synchronisation, no allocation: CUDA-graph capturable. */
+AHV_API int ahv_scores_exchange(const float* part, int B, int64_t N, float* scores, int rank, int world, void* const* peers,
+                                int peer_max_pairs, int peer_max_k, int64_t peer_max_hyps, void* stream);
+
+/* ahv_refine_gradient_distinct over a hypothesis set sharded across the GPUs of one node (extension).  Every rank
+ * passes the WHOLE rotation set R (and the same volumes and arguments) and receives the whole-set result: every
+ * output equals ahv_refine_gradient_distinct's on one GPU over the same set, bit for bit, on every rank.  Rank r
+ * scores hypotheses [lo, hi) (the partition of ahv_scores_exchange).
+ *   min_sep_deg == 0: the slice's top-k, merged over the ranks by the top-k exchange (ahv_verify_sharded).
+ *   min_sep_deg > 0:  the slice's scores, all-gathered by ahv_scores_exchange, then ahv_topk_distinct over the
+ *                     whole [B,N] and R on EVERY rank.  This selection is replicated, not sharded: greedy
+ *                     suppression does not compose from per-shard lists (a rotation that wins on its shard may
+ *                     suppress a neighbour and then lose to another shard's winner, and the neighbour it suppressed
+ *                     belonged to the global answer).  Needs N <= peer_max_hyps.
+ * The rank then ascends items [ilo, ihi) of the B*k (pair, slot) items, the same partition over B*k (k < world and
+ * ranks with no item are fine), and one exchange gives every rank every ascended slot; the per-pair arg-max and its
+ * rotation are computed on every rank.  Empty distinct slots: R_all NaN, score_all -inf, as on one GPU.
+ * k <= min(32, N), B <= peer_max_pairs, k <= peer_max_k; every rank must make the same call.  world == 1 is
+ * ahv_refine_gradient(_distinct) (peers may be NULL).  Two exchanges per call for world > 1.  Workspace:
+ * ahv_refine_gradient_sharded_workspace_bytes(B, N, k, world).  No host synchronisation, no allocation: CUDA-graph
+ * capturable. */
+AHV_API size_t ahv_refine_gradient_sharded_workspace_bytes(int B, int64_t N, int k, int world);
+AHV_API int ahv_refine_gradient_sharded(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R,
+                                        int r_per_pair, const float* W1, const float* W2, const float* b2, const float* base,
+                                        int k, int steps, float step_deg, float min_sep_deg, float* first_val,
+                                        int64_t* first_idx, float* first_R, float* R_all, float* score_all, float* best_val,
+                                        int64_t* best_idx, float* R_best, int B, int64_t N, int math_mode, void* workspace,
+                                        size_t workspace_bytes, int rank, int world, void* const* peers, int peer_max_pairs,
+                                        int peer_max_k, int64_t peer_max_hyps, void* stream);
+
 /* Entries taking HOST buffers (pageable or pinned) - what a non-PyTorch host (ctypes / cgo / JNI) binds: copy
  * the inputs to the device, run the whole verification step (ahv_verify, or ahv_verify_sharded when world > 1)
  * and copy the selection back; `stream` is synchronised before returning.  vol_tgt_host [B,16,8,8,8] fp32;
