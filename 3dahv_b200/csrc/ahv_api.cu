@@ -497,6 +497,30 @@ AHV_API int ahv_topk_distinct(const float* scores, const float* R, int r_per_pai
                               (cudaStream_t)stream);
 }
 
+// ---- posterior mass of the selected rotations under the verifier's softmax (extension) -------------------
+namespace {
+bool posterior_sizes_ok(int B, int64_t N, int k) { return B >= 0 && N >= 1 && n_ok(N) && k >= 0 && k <= kMaxK; }
+}  // namespace
+
+AHV_API size_t ahv_posterior_mass_workspace_bytes(int B, int64_t N, int k) {
+  return posterior_sizes_ok(B, N, k) ? posterior_workspace_bytes(B, N, k) : 0;
+}
+
+AHV_API int ahv_posterior_mass(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N,
+                               int k, float radius_deg, float temperature, float* log_z, float* mass, void* workspace,
+                               size_t workspace_bytes, void* stream) {
+  if (!posterior_sizes_ok(B, N, k) || !min_sep_ok(radius_deg)) return AHV_EINVAL;
+  if (!std::isfinite(temperature) || !(temperature > 0.0f)) return AHV_EINVAL;
+  if (B > 0 && !all_set(scores, R, log_z, workspace)) return AHV_EINVAL;
+  if (k > 0 ? (B > 0 && !all_set(centers, mass)) : (centers || mass)) return AHV_EINVAL;  // k == 0: log_z alone
+  if (!all_aligned16(R, centers, workspace)) return AHV_EINVAL;
+  if (B > 0 && workspace_bytes < posterior_workspace_bytes(B, N, k)) return AHV_EWORKSPACE;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  return launch_posterior_mass(scores, R, r_per_pair != 0, centers, B, N, k, radius_deg, temperature, log_z, mass, workspace,
+                               (cudaStream_t)stream);
+}
+
 // ---- hypothesis set sharded over the GPUs of one node: winners exchanged through peer memory -------------
 AHV_API size_t ahv_peer_bytes(int max_pairs, int max_k) {
   return (max_pairs < 1 || !k_ok(max_k)) ? 0 : peer::buffer_bytes(max_pairs, max_k);

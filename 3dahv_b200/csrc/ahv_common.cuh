@@ -255,5 +255,8 @@ int launch_gather_rotations(const float* R, int r_per_pair, const int64_t* idx, 
                             int B, int64_t N, int k, float* R_out, cudaStream_t s);
 int launch_topk_distinct(const float* scores, const float* R, int r_per_pair, int B, int64_t N, int k, float min_sep_deg,
                          float* val, int64_t* idx, float* R_best, cudaStream_t s);
+size_t posterior_workspace_bytes(int B, int64_t N, int k);
+int launch_posterior_mass(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N, int k,
+                          float radius_deg, float temperature, float* log_z, float* mass, void* ws, cudaStream_t s);
 
 }  // namespace ahv

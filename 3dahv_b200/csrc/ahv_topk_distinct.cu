@@ -44,6 +44,15 @@ __device__ __forceinline__ u64 warp_max64(u64 v) {
   return v;
 }
 
+// t(a, w) = trace(R_a R_w^T): nine __fmul_rn products summed left to right with __fadd_rn (no contraction).  The one
+// definition of the trace that the distinct selection and the posterior mass (ahv_posterior_mass) both test.
+__device__ __forceinline__ float trace_rn(const float (&a)[9], const float* w) {
+  float t = __fmul_rn(a[0], w[0]);
+#pragma unroll
+  for (int e = 1; e < 9; ++e) t = __fadd_rn(t, __fmul_rn(a[e], w[e]));
+  return t;
+}
+
 // t(n, w_i) < c for every winner i in [from, to)
 __device__ __forceinline__ bool separated(const float* __restrict__ Rn, const float (*win)[9], int from, int to, float c) {
   float a[9];
@@ -51,10 +60,7 @@ __device__ __forceinline__ bool separated(const float* __restrict__ Rn, const fl
   for (int e = 0; e < 9; ++e) a[e] = __ldg(Rn + e);
 #pragma unroll 1
   for (int i = from; i < to; ++i) {
-    float t = __fmul_rn(a[0], win[i][0]);
-#pragma unroll
-    for (int e = 1; e < 9; ++e) t = __fadd_rn(t, __fmul_rn(a[e], win[i][e]));
-    if (!(t < c)) return false;
+    if (!(trace_rn(a, win[i]) < c)) return false;
   }
   return true;
 }
@@ -150,6 +156,13 @@ topk_distinct_kernel(const float* __restrict__ scores, const float* __restrict__
   }
   cluster.sync();  // no CTA leaves while another may still read its partials
 }
+// c = fp32(1 + 2 cos(theta)), evaluated in double and rounded once: t(a, b) >= c <=> the rotations lie within theta
+// of each other (up to the rounding of t).  theta >= 180 gives -inf: every rotation lies within 180 degrees (the
+// distinct selection does not test then, it keeps w_0 alone).
+inline float trace_threshold(float theta_deg) {
+  if (theta_deg >= 180.0f) return -INFINITY;
+  return (float)(1.0 + 2.0 * std::cos((double)theta_deg * 3.14159265358979323846 / 180.0));
+}
 }  // namespace distinct
 
 int launch_topk_distinct(const float* scores, const float* R, int r_per_pair, int B, int64_t N, int k, float min_sep_deg,
@@ -157,7 +170,7 @@ int launch_topk_distinct(const float* scores, const float* R, int r_per_pair, in
   using namespace distinct;
   if (B == 0) return AHV_OK;
   const bool suppress = min_sep_deg > 0.0f;
-  const float c = (float)(1.0 + 2.0 * std::cos((double)min_sep_deg * 3.14159265358979323846 / 180.0));
+  const float c = trace_threshold(min_sep_deg);
   const int rounds = min_sep_deg >= 180.0f ? 1 : k;
   const int64_t slice = (N + kCtas - 1) / kCtas;
   const bool staged = slice * (int64_t)(sizeof(float) + 1) <= kDynSmemBytes;  // N up to ~370 000
@@ -167,6 +180,194 @@ int launch_topk_distinct(const float* scores, const float* R, int r_per_pair, in
   const unsigned clusters = (unsigned)(B < 65535 ? B : 65535);
   topk_distinct_kernel<<<dim3(kCtas, clusters), kThreads, smem, s>>>(scores, R, r_per_pair, B, N, k, rounds, suppress, c,
                                                                      staged, tracked, val, idx, R_best);
+  AHV_CUDA_OK(cudaGetLastError());
+  return AHV_OK;
+}
+
+// Posterior mass of the selected rotations (ahv_posterior_mass; DESIGN.md §4.7) under p_b(n) = e^{s[b,n]/T} / Z_b:
+//   log_z[b]   = m/T + log sum_n exp((s[b,n] - m)/T),  m = max_n s[b,n]
+//   mass[b,j]  = sum_{n -> j} exp((s - m)/T) / sum_n exp((s - m)/T),
+// where n -> j for the lowest slot j with t(n, c_j) >= c (trace_rn and trace_threshold above, so with the distinct
+// winners as centres and theta = min_sep, slot j holds the winner and exactly the hypotheses it suppressed).
+//
+// Two launches, deterministic: the hypotheses of a pair are cut into chunks of kChunk (a constant, so the summation
+// order depends on N alone, not on B or on the SM count).  Pass 1, grid (chunk, pair): the chunk's maximum m_c and,
+// in double, S_c = sum exp((s - m_c)/T) and each slot's share, per thread in index order, then warp butterflies and
+// warps in order; a chunk holding a NaN or +inf score records m_c = NaN.  Pass 2, one CTA per pair: m = max m_c
+// (exact), then every sum rescaled by exp((m_c - m)/T) and added over the chunks in a fixed tree, each cast to fp32
+// once.  Workspace: [the chunk sums, B*chunks*(k+1) doubles | the chunk maxima, B*chunks floats].
+namespace posterior {
+constexpr int kThreads = 128;
+constexpr int kWarps = kThreads / 32;
+constexpr int kPer = 16;                      // hypotheses per thread of a chunk
+constexpr int64_t kChunk = kThreads * kPer;   // 2048
+constexpr int kFinalThreads = 256;
+
+__device__ __forceinline__ double warp_sum_d(double v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+
+__global__ void __launch_bounds__(kThreads)
+posterior_chunk_kernel(const float* __restrict__ scores, const float* __restrict__ R, int r_per_pair,
+                       const float* __restrict__ centers, int B, int64_t N, int k, float c, double T, int chunks,
+                       double* __restrict__ ws_sum, float* __restrict__ ws_max) {
+  __shared__ double s_acc[kMaxK * kThreads];  // slot j of thread t at [j][t]: each thread adds into its own column
+  __shared__ double s_red[kMaxK + 1][kWarps];
+  __shared__ float s_cen[kMaxK][9];
+  __shared__ float s_wmax[kWarps];
+  __shared__ int s_wbad[kWarps];
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  const int64_t first = (int64_t)blockIdx.x * kChunk;
+  for (int b = blockIdx.y; b < B; b += gridDim.y) {
+    const float* row = scores + (size_t)b * N;
+    const float* Rp = R + (r_per_pair ? (size_t)b * N * 9 : 0);
+    float s[kPer];
+    float mx = -INFINITY;
+    bool bad = false;
+#pragma unroll
+    for (int i = 0; i < kPer; ++i) {
+      const int64_t n = first + i * kThreads + t;
+      s[i] = n < N ? __ldg(row + n) : -INFINITY;
+      bad |= isnan(s[i]) || s[i] == INFINITY;
+      mx = fmaxf(mx, s[i]);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+    bad = __any_sync(0xffffffffu, bad);
+    if (lane == 0) {
+      s_wmax[warp] = mx;
+      s_wbad[warp] = bad;
+    }
+    for (int e = t; e < k * 9; e += kThreads) s_cen[e / 9][e % 9] = __ldg(centers + (size_t)b * k * 9 + e);
+    for (int j = 0; j < k; ++j) s_acc[j * kThreads + t] = 0.0;
+    __syncthreads();
+#pragma unroll
+    for (int w = 0; w < kWarps; ++w) {
+      mx = fmaxf(mx, s_wmax[w]);
+      bad |= s_wbad[w] != 0;
+    }
+    double tot = 0.0;
+    if (!bad) {
+#pragma unroll
+      for (int i = 0; i < kPer; ++i) {
+        if (s[i] == -INFINITY) continue;  // contributes 0 (and every score of the chunk may be -inf: no inf - inf)
+        const double e = exp(((double)s[i] - (double)mx) / T);
+        tot += e;
+        if (k > 0) {
+          const float* Rn = Rp + (size_t)(first + i * kThreads + t) * 9;
+          float a[9];
+#pragma unroll
+          for (int q = 0; q < 9; ++q) a[q] = __ldg(Rn + q);
+#pragma unroll 1
+          for (int j = 0; j < k; ++j) {
+            if (distinct::trace_rn(a, s_cen[j]) >= c) {  // a NaN trace (empty slot) never passes
+              s_acc[j * kThreads + t] += e;
+              break;
+            }
+          }
+        }
+      }
+    }
+    for (int v = 0; v <= k; ++v) {
+      const double x = warp_sum_d(v == 0 ? tot : s_acc[(v - 1) * kThreads + t]);
+      if (lane == 0) s_red[v][warp] = x;
+    }
+    __syncthreads();
+    const size_t rec = (size_t)b * chunks + blockIdx.x;
+    if (t <= k) {
+      double x = s_red[t][0];
+#pragma unroll
+      for (int w = 1; w < kWarps; ++w) x += s_red[t][w];
+      ws_sum[rec * (k + 1) + t] = x;
+    }
+    if (t == 0) ws_max[rec] = bad ? NAN : mx;
+    __syncthreads();  // the next pair reuses the shared arrays
+  }
+}
+
+__global__ void __launch_bounds__(kFinalThreads)
+posterior_final_kernel(const double* __restrict__ ws_sum, const float* __restrict__ ws_max, int chunks, int k, double T,
+                       float* __restrict__ log_z, float* __restrict__ mass) {
+  constexpr int kW = kFinalThreads / 32;
+  __shared__ float s_wmax[kW];
+  __shared__ int s_wbad[kW];
+  __shared__ double s_red[kMaxK + 1][kW];
+  const int b = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  const float* mc = ws_max + (size_t)b * chunks;
+  const double* sc = ws_sum + (size_t)b * chunks * (k + 1);
+  float m = -INFINITY;
+  bool bad = false;
+  for (int i = t; i < chunks; i += kFinalThreads) {
+    const float x = mc[i];
+    bad |= isnan(x);
+    m = fmaxf(m, x);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  bad = __any_sync(0xffffffffu, bad);
+  if (lane == 0) {
+    s_wmax[warp] = m;
+    s_wbad[warp] = bad;
+  }
+  __syncthreads();
+#pragma unroll
+  for (int w = 0; w < kW; ++w) {
+    m = fmaxf(m, s_wmax[w]);
+    bad |= s_wbad[w] != 0;
+  }
+  // every score -inf: Z = 0, log_z = -inf and the masses 0/0 = NaN
+  const bool live = !bad && m != -INFINITY;
+  for (int v = 0; v <= k; ++v) {
+    double x = 0.0;
+    if (live) {
+      for (int i = t; i < chunks; i += kFinalThreads) {
+        const float mi = mc[i];
+        if (mi != -INFINITY) x += sc[(size_t)i * (k + 1) + v] * exp(((double)mi - (double)m) / T);
+      }
+    }
+    x = warp_sum_d(x);
+    if (lane == 0) s_red[v][warp] = x;
+  }
+  __syncthreads();
+  if (t <= k) {
+    double S = s_red[t][0], Z = s_red[0][0];
+#pragma unroll
+    for (int w = 1; w < kW; ++w) {
+      S += s_red[t][w];
+      Z += s_red[0][w];
+    }
+    if (t == 0) log_z[b] = bad ? NAN : (float)((double)m / T + log(S));
+    else mass[(size_t)b * k + t - 1] = bad ? NAN : (float)(S / Z);
+  }
+}
+
+struct Ws {
+  int chunks;
+  size_t max, total;  // byte offsets: the sums at 0, the maxima at `max`
+  Ws(int B, int64_t N, int k)
+      : chunks((int)((N + kChunk - 1) / kChunk)),
+        max(((size_t)B * chunks * (k + 1) * sizeof(double) + 255) / 256 * 256),
+        total(max + ((size_t)B * chunks * sizeof(float) + 255) / 256 * 256) {}
+};
+}  // namespace posterior
+
+size_t posterior_workspace_bytes(int B, int64_t N, int k) { return posterior::Ws(B, N, k).total; }
+
+int launch_posterior_mass(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N, int k,
+                          float radius_deg, float temperature, float* log_z, float* mass, void* ws, cudaStream_t s) {
+  using namespace posterior;
+  if (B == 0) return AHV_OK;
+  const Ws w(B, N, k);
+  double* ws_sum = static_cast<double*>(ws);
+  float* ws_max = reinterpret_cast<float*>(static_cast<unsigned char*>(ws) + w.max);
+  const unsigned pairs = (unsigned)(B < 65535 ? B : 65535);
+  posterior_chunk_kernel<<<dim3((unsigned)w.chunks, pairs), kThreads, 0, s>>>(
+      scores, R, r_per_pair, centers, B, N, k, distinct::trace_threshold(radius_deg), (double)temperature, w.chunks, ws_sum,
+      ws_max);
+  AHV_CUDA_OK(cudaGetLastError());
+  posterior_final_kernel<<<(unsigned)B, kFinalThreads, 0, s>>>(ws_sum, ws_max, w.chunks, k, (double)temperature, log_z, mass);
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }

@@ -605,6 +605,39 @@ def topk_distinct(scores: torch.Tensor, R: torch.Tensor, k: int, min_sep_deg: fl
     return val, idx, Rb
 
 
+def posterior_mass_workspace_bytes(B: int, N: int, k: int) -> int:
+    """Bytes of scratch `posterior_mass` needs (0 for invalid sizes)."""
+    return int(_lib.lib().ahv_posterior_mass_workspace_bytes(B, N, k))
+
+
+def posterior_mass(scores: torch.Tensor, R: torch.Tensor, centers: torch.Tensor | None, radius_deg: float,
+                   temperature: float = 0.1, workspace: torch.Tensor | None = None):
+    """ahv_posterior_mass: the softmax p_b(n) = exp(scores[b,n]/T) / Z_b over the hypothesis set, summarised per pair.
+    Returns (log_z [B] = log Z_b, mass [B,k]): mass[b,j] is the probability of the hypotheses whose lowest slot j with
+    trace(R_n c_j^T) >= fp32(1 + 2 cos(radius_deg)) is j - `topk_distinct`'s trace test, so with centers = its R_best
+    and radius_deg = its min_sep_deg, slot j holds its winner and the hypotheses that winner suppressed.  scores [B,N];
+    R [N,3,3] or [B,N,3,3]; centers [B,k,3,3] (NaN = empty slot, mass 0) or None (k = 0: mass is [B,0]).  A pair with a
+    NaN or +inf score gets NaN outputs.  Deterministic, bit-identical whatever the batch around a pair."""
+    s, R = _dev(scores, "scores"), _dev(R, "R")
+    B, N = s.shape
+    per_pair = R.dim() == 4
+    if tuple(R.shape) != ((B, N, 3, 3) if per_pair else (N, 3, 3)):
+        raise ValueError("R must be [N,3,3] or [B,N,3,3] for scores [B,N]")
+    c = None
+    if centers is not None:
+        c = _dev(centers, "centers")
+        if c.dim() != 4 or c.shape[0] != B or tuple(c.shape[2:]) != (3, 3):
+            raise ValueError("centers must be [B,k,3,3]")
+    k = 0 if c is None else c.shape[1]
+    log_z = torch.empty(B, device=s.device, dtype=torch.float32)
+    mass = torch.empty(B, k, device=s.device, dtype=torch.float32)
+    workspace, ws_bytes = _workspace(workspace, posterior_mass_workspace_bytes(B, N, k), s.device)
+    _call("ahv_posterior_mass", s.device, s.data_ptr(), R.data_ptr(), int(per_pair), c.data_ptr() if k else None, B, N, k,
+          float(radius_deg), float(temperature), log_z.data_ptr(), mass.data_ptr() if k else None, workspace.data_ptr(),
+          ws_bytes)
+    return log_z, mass
+
+
 def topk_merge(vals: torch.Tensor, idx: torch.Tensor):
     """Merge [parts,B,k] shard lists into [B,k] (same ordering rule)."""
     v, i = _dev(vals, "vals"), _dev(idx, "idx", torch.int64)

@@ -41,6 +41,40 @@ class VerifyResult:
     R_best: torch.Tensor           # [B,k,3,3] sampled_R[pred_index] (:196)
 
 
+@dataclass
+class Posterior:
+    """The selection and what the verifier's softmax p_b(n) = exp(s[b,n]/T) / Z_b says about it (`posterior`)."""
+    topk_val: torch.Tensor                # [B,k]
+    topk_idx: torch.Tensor                # [B,k] int64 (-1: empty distinct slot)
+    R_best: torch.Tensor                  # [B,k,3,3] (NaN: empty distinct slot)
+    mass: torch.Tensor                    # [B,k] probability held by each selected rotation's neighbourhood
+    log_z: torch.Tensor                   # [B] log Z_b
+    log_density: torch.Tensor | None      # [B,Q] log-density of R_query w.r.t. the normalised Haar measure
+
+
+def _posterior_radius(min_sep_deg: float, radius_deg: float | None) -> float:
+    if radius_deg is not None:
+        return radius_deg
+    if not min_sep_deg > 0:
+        raise ValueError("radius_deg is required when min_sep_deg is 0")
+    return min_sep_deg
+
+
+def _posterior(scores, R, k, min_sep_deg, radius_deg, temperature, s_query) -> Posterior:
+    """The selection (`ops.topk` or `ops.topk_distinct`) and `ops.posterior_mass` over a whole [B,N] score matrix."""
+    if min_sep_deg > 0:
+        val, idx, R_best = ops.topk_distinct(scores, R, k, min_sep_deg)
+    else:
+        val, idx = ops.topk(scores, k)
+        R_best = ops.gather_rotations(R, idx)
+    log_z, mass = ops.posterior_mass(scores, R, R_best, radius_deg, temperature)
+    log_density = None
+    if s_query is not None:
+        N = scores.shape[1]
+        log_density = (s_query.double() / temperature - log_z.double()[:, None] + math.log(N)).float()
+    return Posterior(val, idx, R_best, mass, log_z, log_density)
+
+
 class HypothesisVerifier:
     """Holds the verification-head weights (state-dict names
     `feature_aligner.feature_embedding_2d.{0.weight,2.weight,2.bias}`)."""
@@ -105,6 +139,34 @@ class HypothesisVerifier:
                                      return_scores=return_scores, workspace=ws)
         R_best = ops.gather_rotations(R, idx, idx_offset) if gather else None
         return VerifyResult(scores, val, idx, R_best)
+
+    @torch.no_grad()
+    def posterior(self, vol_src, vol_tgt, R, k: int = 1, min_sep_deg: float = 0.0, radius_deg: float | None = None,
+                  temperature: float = 0.1, R_query=None) -> Posterior:
+        """The selection of `score` (the top-k, or with min_sep_deg > 0 the top-k of distinct rotations) and how much of
+        the verifier's softmax p_b(n) = exp(s[b,n]/T) / Z_b over the set it holds.  T = 0.1 is the InfoNCE training
+        temperature (modules/model.py:43-63), under which p_b is the model's own estimate of where the rotation lies.
+        `mass[b,j]`: the probability of the hypotheses within radius_deg of slot j's rotation and of no earlier slot
+        (`ops.posterior_mass`); radius_deg defaults to min_sep_deg, where slot j holds its winner and the hypotheses
+        that winner suppressed.  With radius_deg = ACC_THR and k = 1, mass[b,0] is the model's estimate that the
+        prediction is correct at ACC_THR; 1 - mass.sum(1) is the probability no slot holds.
+        `R_query` [B,Q,3,3] (e.g. the ground truth as Q = 1): `log_density` [B,Q] = s_q/T - log Z_b + log N, the
+        log-density of p_b at R_query w.r.t. the normalised Haar measure (SO(3) has volume 1), meaningful when the set
+        is Haar-random or near-uniform.  Subtract log(pi^2) for the convention that takes the volume of SO(3) as pi^2.
+        vol_src/vol_tgt [B,16,8,8,8]; R [N,3,3] shared or [B,N,3,3] per pair.  No host synchronisation."""
+        radius_deg = _posterior_radius(min_sep_deg, radius_deg)
+        dev = vol_src.device
+        W1, W2, b2 = self._weights_on(dev)
+        k, N = _clamp_k(k, R)
+        if N == 0:
+            raise ValueError("empty hypothesis set")
+        vs = _src_volume(vol_src)
+        tf = self.target_features(vol_tgt)
+        scores = ops.score(vs, tf, R, W1, W2, b2, k=0, math=self.math, workspace=self._workspace(vol_src.shape[0], N, 1, dev))[0]
+        s_query = None
+        if R_query is not None:
+            s_query = ops.score(vs, tf, R_query, W1, W2, b2, k=0, math=self.math)[0]
+        return _posterior(scores, R, k, min_sep_deg, radius_deg, temperature, s_query)
 
     @torch.no_grad()
     def predict(self, vol_src, vol_tgt, R):

@@ -313,6 +313,26 @@ AHV_API int ahv_refine_gradient_distinct(const void* vol_src, int vol_dtype, con
 AHV_API int ahv_topk_distinct(const float* scores, const float* R, int r_per_pair, int B, int64_t N, int k,
                               float min_sep_deg, float* topk_val, int64_t* topk_idx, float* R_best, void* stream);
 
+/* Posterior mass of selected rotations (extension): the verification scores are trained as the logits of a
+ * distribution over SO(3) (InfoNCE, modules/model.py:43-63), p_b(n) = exp(s[b,n]/T) / Z_b.  With m = max_n s[b,n]:
+ *   log_z[b]  = m/T + log sum_n exp((s[b,n] - m)/T)
+ *   mass[b,j] = sum_{n -> j} exp((s[b,n] - m)/T) / sum_n exp((s[b,n] - m)/T)
+ * where hypothesis n goes to the LOWEST slot j with t(n, c_j) >= c: t and c = fp32(1 + 2 cos(radius_deg * pi / 180))
+ * are ahv_topk_distinct's (radius_deg == 180: every rotation qualifies).  With centers = ahv_topk_distinct's R_best and
+ * radius_deg = its min_sep_deg, slot j's mass is its winner plus exactly the hypotheses that winner suppressed;
+ * 1 - sum_j mass[b,j] is the mass no slot holds.  scores [B,N]; R [N,3,3] (r_per_pair == 0) or [B,N,3,3]; centers
+ * [B,k,3,3], a NaN centre being an empty slot (mass 0); log_z [B], mass [B,k].  0 <= k <= 32 (k == 0: centers and
+ * mass NULL, log_z alone), 1 <= N <= 2^31 - 1, 0 <= radius_deg <= 180, temperature finite and > 0; R, centers and the
+ * workspace 16-byte aligned.  A -inf score contributes 0; a pair with a NaN or +inf score gets NaN outputs; a pair whose
+ * scores are all -inf gets log_z = -inf and NaN masses.  Sums run in double in a fixed order and are cast to fp32
+ * once: the bits depend on the inputs alone (not on B, the pair's place in the batch or the SM count).  Two launches,
+ * workspace ahv_posterior_mass_workspace_bytes(B, N, k) (~B * ceil(N/2048) * (k+1) * 8 bytes), no allocation, no host
+ * synchronisation: CUDA-graph capturable. */
+AHV_API size_t ahv_posterior_mass_workspace_bytes(int B, int64_t N, int k);
+AHV_API int ahv_posterior_mass(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N,
+                               int k, float radius_deg, float temperature, float* log_z, float* mass, void* workspace,
+                               size_t workspace_bytes, void* stream);
+
 /* torch.max / top-k over an existing score matrix (modules/model.py:195). */
 AHV_API int ahv_topk(const float* scores, int B, int64_t N, int k, int64_t idx_offset, float* topk_val,
              int64_t* topk_idx, void* workspace, size_t workspace_bytes, void* stream);
