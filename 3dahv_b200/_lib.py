@@ -41,6 +41,8 @@ SIGNATURES = {
     "ahv_forward_3d2d": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _vp]),
     "ahv_workspace_bytes": (_sz, [_i, _i64, _i]),
     "ahv_score": (_i, [_vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _i64, _i, _vp, _sz, _vp]),
+    "ahv_verify_screen_stats": (_i, [_vp, _i, _i64, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int),
+                                     ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_float)]),
     "ahv_verify": (_i, [_vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _i64, _i, _vp, _sz, _vp]),
     "ahv_refine_workspace_bytes": (_sz, [_i, _i64, _i, _i]),
     "ahv_refine": (_i, [_vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, ctypes.c_float, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp,

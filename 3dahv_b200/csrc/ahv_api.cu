@@ -73,6 +73,17 @@ struct ShardedRefineWs {
         total(top + align_up(topk_workspace_bytes(B, k, 1), 256)) {}
 };
 
+// The screened arg-max (launch_verify_tc_screened, ahv_score_tc.cu) serves ahv_verify and ahv_verify_sharded for fp32
+// volumes under AHV_MATH_TC with k == 1 and no scores returned, once a call has enough items to repay its five extra
+// launches (the single-pair latency calls, B = 1 at N = 3 000 or 50 000, stay on the single pass).  Its buffers live in the
+// verification workspace that the k == 1 path leaves unused - the scores (B*N fp32) and the top-k partials (B*N/16
+// bytes and more) - so the workspace size is the same as before; that needs N of about 40 000 or more.
+constexpr int64_t kScreenMinItems = 1 << 18;
+bool screened(const VerifyWs& w, int vol_dtype, int math_mode, const float* scores, int k, int B, int64_t N) {
+  return vol_dtype == AHV_VOL_F32 && math_mode == AHV_MATH_TC && k == 1 && !scores && (int64_t)B * N >= kScreenMinItems &&
+         N * sizeof(float) >= kScreenList * 10 * sizeof(float) && w.tc - w.topk >= ScreenLists::bytes(B);
+}
+
 // dist.shard_bounds: rank's contiguous share [lo, hi) of n items
 void shard_bounds(int64_t n, int rank, int world, int64_t* lo, int64_t* hi) {
   const int64_t per = (n + world - 1) / world;
@@ -271,6 +282,20 @@ AHV_API size_t ahv_workspace_bytes(int B, int64_t N, int k) {
   return B < 0 || N < 0 ? 0 : VerifyWs(B, N, k).total;
 }
 
+AHV_API int ahv_verify_screen_stats(const void* workspace, int B, int64_t N, int* is_screened, int* flagged_pairs,
+                                    int* contenders, float* max_err) {
+  if (B < 0 || !n_ok(N) || !is_screened) return AHV_EINVAL;
+  const VerifyWs w(B, N, 1);
+  *is_screened = screened(w, AHV_VOL_F32, AHV_MATH_TC, nullptr, 1, B, N);
+  if (!*is_screened || (!flagged_pairs && !contenders && !max_err)) return AHV_OK;
+  if (!workspace) return AHV_EINVAL;
+  const ScreenLists L(static_cast<unsigned char*>(const_cast<void*>(workspace)) + w.topk, B);
+  if (flagged_pairs) AHV_CUDA_OK(cudaMemcpy(flagged_pairs, L.flagged, sizeof(int), cudaMemcpyDeviceToHost));
+  if (contenders) AHV_CUDA_OK(cudaMemcpy(contenders, L.count, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost));
+  if (max_err) AHV_CUDA_OK(cudaMemcpy(max_err, L.err, (size_t)B * sizeof(float), cudaMemcpyDeviceToHost));
+  return AHV_OK;
+}
+
 AHV_API int ahv_topk(const float* scores, int B, int64_t N, int k, int64_t idx_offset, float* topk_val,
              int64_t* topk_idx, void* workspace, size_t workspace_bytes, void* stream) {
   if (B < 0 || !n_ok(N) || !k_ok(k)) return AHV_EINVAL;
@@ -344,6 +369,10 @@ AHV_API int ahv_verify(const void* vol_src, int vol_dtype, const float* vol_tgt,
   if (!workspace || workspace_bytes < w.total) return AHV_EWORKSPACE;
   cudaStream_t s = (cudaStream_t)stream;
   void* ws_tc = static_cast<unsigned char*>(workspace) + w.tc;  // packed weights, target features, scales, keys
+  if (screened(w, vol_dtype, math_mode, scores, k, B, N))
+    return launch_verify_tc_screened(static_cast<const float*>(vol_src), vol_tgt, R, r_per_pair != 0, W1, W2, b2, base,
+                                     topk_val, topk_idx, R_best, idx_offset, B, N, ws_tc, workspace_bytes - w.tc,
+                                     static_cast<float*>(workspace), static_cast<unsigned char*>(workspace) + w.topk, s);
   if (math_mode != AHV_MATH_FP32 && k == 1)  // three launches, nothing but 40 B per hypothesis touches HBM
     return launch_verify_tc_argmax(vol_src, vol_dtype, vol_tgt, R, r_per_pair != 0, W1, W2, b2, base, scores,
                                    topk_val, topk_idx, R_best, idx_offset, B, N, ws_tc,
@@ -660,6 +689,10 @@ AHV_API int ahv_verify_sharded(const void* vol_src, int vol_dtype, const float* 
   if (!workspace || workspace_bytes < w.total) return AHV_EWORKSPACE;
   unsigned char* ws = static_cast<unsigned char*>(workspace);
   cudaStream_t s = (cudaStream_t)stream;
+  if (N > 0 && screened(w, vol_dtype, math_mode, nullptr, k, B, N))  // its last pass exchanges and merges the winners
+    return launch_verify_tc_screened(static_cast<const float*>(vol_src), vol_tgt, R, r_per_pair != 0, W1, W2, b2, base,
+                                     topk_val, topk_idx, R_best, idx_offset, B, N, ws + w.tc, w.lists - w.tc,
+                                     reinterpret_cast<float*>(ws), ws + w.topk, s, &pa);
   if (k == 1 && N > 0 && math_mode != AHV_MATH_FP32)  // the scoring kernel exchanges and merges the winners itself
     return launch_verify_tc_argmax(vol_src, vol_dtype, vol_tgt, R, r_per_pair != 0, W1, W2, b2, base, nullptr, topk_val,
                                    topk_idx, R_best, idx_offset, B, N, ws + w.tc, w.lists - w.tc, s,

@@ -237,6 +237,10 @@ int launch_verify_tc_argmax(const void* vol_src, int vol_dtype, const float* vol
                             const float* base, float* scores, float* best_val, int64_t* best_idx,
                             float* R_best, int64_t idx_offset, int B, int64_t N, void* ws, size_t ws_bytes,
                             cudaStream_t s, bool f16_gather, const peer::Args* pa = nullptr);
+int launch_verify_tc_screened(const float* vol_src, const float* vol_tgt, const float* R, int r_per_pair, const float* W1,
+                              const float* W2, const float* b2, const float* base, float* best_val, int64_t* best_idx,
+                              float* R_best, int64_t idx_offset, int B, int64_t N, void* ws, size_t ws_bytes, float* s16,
+                              void* lists, cudaStream_t s, const peer::Args* pa = nullptr);
 int launch_topk_exchange(const float* val, const int64_t* idx, const float* R, int r_per_pair, int64_t idx_offset,
                          int64_t N, int B, int k, float* out_val, int64_t* out_idx, float* R_best,
                          const peer::Args& pa, cudaStream_t s);
@@ -255,6 +259,35 @@ int launch_gather_rotations(const float* R, int r_per_pair, const int64_t* idx, 
                             int B, int64_t N, int k, float* R_out, cudaStream_t s);
 int launch_topk_distinct(const float* scores, const float* R, int r_per_pair, int B, int64_t N, int k, float min_sep_deg,
                          float* val, int64_t* idx, float* R_best, cudaStream_t s);
+// Screened arg-max of ahv_verify (k = 1, fp32 volumes, AHV_MATH_TC; the passes are described at
+// launch_verify_tc_screened in ahv_score_tc.cu).  Per pair a list of kScreenList hypotheses: the contenders (16-bit
+// gather score within 2 tau of the pair's screened maximum, at most kScreenCap of them, padded with the first), then
+// kScreenProbes fixed strided probes.  tau is in score units (scores are means of cosines): 27x the largest 16-bit vs
+// fp32 gather difference on the bench workload (7.3e-5) and at least 8x that of order-one volumes with outliers up to
+// 3e7 times the bulk, of the mixed per-pair scales and of the head-weight cases short of one W1 row dominating the
+// others by 2^6 (profiles/r11_screen_margin.json); with it the bench workload has at most 22 contenders per pair.
+constexpr int kScreenCap = 224;
+constexpr int kScreenProbes = 32;
+constexpr int kScreenList = kScreenCap + kScreenProbes;
+constexpr float kScreenTau = 2e-3f;
+struct ScreenLists {  // carved from the verification workspace's top-k partials region (unused when k == 1)
+  int* idx;      // [B][kScreenList] hypothesis index
+  float* s16;    // [B][kScreenList] its 16-bit gather score
+  int* count;    // [B] contenders found (more than kScreenCap: the pair is flagged)
+  float* err;    // [B] largest |fp32 score - 16-bit score| over the list
+  int* flagged;  // [1 + B]: number of flagged pairs, then the flagged pairs (in no particular order)
+  static size_t bytes(int B) { return (size_t)B * kScreenList * 8 + (size_t)B * 8 + (size_t)(B + 1) * 4; }
+  ScreenLists(void* p, int B) {
+    idx = static_cast<int*>(p);
+    s16 = reinterpret_cast<float*>(idx + (size_t)B * kScreenList);
+    count = reinterpret_cast<int*>(s16 + (size_t)B * kScreenList);
+    err = reinterpret_cast<float*>(count + B);
+    flagged = reinterpret_cast<int*>(err + B);
+  }
+};
+int launch_screen_select(const float* s16, const unsigned long long* keys, int B, int64_t N, const float* R, int r_per_pair,
+                         const ScreenLists& L, float* R_list, cudaStream_t s);
+int launch_screen_guard(const float* s32, const ScreenLists& L, int B, unsigned long long* keys, cudaStream_t s);
 size_t posterior_workspace_bytes(int B, int64_t N, int k);
 int launch_posterior_mass(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N, int k,
                           float radius_deg, float temperature, float* log_z, float* mass, void* ws, cudaStream_t s);

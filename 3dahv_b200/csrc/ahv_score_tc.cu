@@ -198,7 +198,8 @@ static int launch_pdl(KernelT kernel, unsigned grid, size_t smem, cudaStream_t s
 template <typename T, bool K16, bool kSave = false>
 int launch_typed(const T* vol_src, const float* vol_tgt, const float* tgt_feat_in, const float* R,
                  int r_per_pair, const float* W1, const float* W2, const float* b2, const float* base,
-                 float* scores, bool want_argmax, int B, int64_t N, const Scratch& sc, Finalize fin, cudaStream_t s) {
+                 float* scores, bool want_argmax, int B, int64_t N, const Scratch& sc, Finalize fin, cudaStream_t s,
+                 const int* pair_list = nullptr) {
   int dev = 0, sms = 0;
   AHV_CUDA_OK(cudaGetDevice(&dev));
   AHV_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
@@ -206,7 +207,7 @@ int launch_typed(const T* vol_src, const float* vol_tgt, const float* tgt_feat_i
   if (prologue) {
     const int st = launch_tgt_feat(vol_tgt, W1, W2, b2, want_argmax ? sc.best_keys : nullptr, sc.tgt_feat, B, s);
     if (st != AHV_OK) return st;
-  } else if (want_argmax) {
+  } else if (want_argmax && !pair_list) {  // a listed-pairs pass adds to the keys (and the cleared counter) it finds
     AHV_CUDA_OK(cudaMemsetAsync(sc.best_keys, 0, (size_t)B * sizeof(u64) + sizeof(unsigned), s));
   }
   fin.counter = sc.counter;
@@ -225,7 +226,7 @@ int launch_typed(const T* vol_src, const float* vol_tgt, const float* tgt_feat_i
   int late = 0;
   if (prologue && kTgtCtasPerPair * (int64_t)B <= grid / 2 && (int64_t)B * N / grid >= 8) late = kTgtCtasPerPair * B;
   return launch_pdl(score_tc_ts_kernel<T, K16, kSave>, grid, MapTS::smem_bytes, s, prologue, vol_map, tgt, R, r_per_pair, b2, base, W1,
-                    W2, scores, keys, B, N, fin, late);
+                    W2, scores, keys, B, N, fin, late, pair_list);
 }
 
 }  // namespace tc
@@ -297,6 +298,24 @@ int launch_score_tc_train(const float* vol_src, const float* tgt_feat, const flo
                                               tc::carve(ws, B), fin, s);
 }
 
+// the fused selection of a k = 1 verification: winners decoded by the scoring kernel's last CTA, or exchanged with the
+// peers' kernels when the set is sharded
+static int make_finalize(float* best_val, int64_t* best_idx, float* R_best, int64_t idx_offset, int B, const peer::Args* pa,
+                         tc::Finalize* fin) {
+  fin->val = best_val;
+  fin->idx = best_idx;
+  fin->R_best = R_best;
+  fin->idx_offset = idx_offset;
+  if (pa && pa->world > 1) {
+    if (pa->world > peer::kMaxPeers || pa->rank < 0 || pa->rank >= pa->world || B > pa->cap_pairs || pa->cap_k < 1)
+      return AHV_EINVAL;
+    for (int r = 0; r < pa->world; ++r)
+      if (!pa->bufs[r]) return AHV_EINVAL;
+    fin->peers = *pa;
+  }
+  return AHV_OK;
+}
+
 // the whole verification step with arg-max selection in two launches: prologue (target features, key
 // clear) -> fused scoring + arg-max, whose last CTA also decodes the winners (no finalize launch)
 int launch_verify_tc_argmax(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R,
@@ -307,20 +326,52 @@ int launch_verify_tc_argmax(const void* vol_src, int vol_dtype, const float* vol
   const int world = pa ? pa->world : 1;
   if ((int64_t)B * N == 0) return world > 1 ? AHV_EINVAL : AHV_OK;  // a sharded step needs every rank in the exchange
   if (ws_bytes < tc::scratch_bytes(B)) return AHV_EWORKSPACE;
-  const tc::Scratch sc = tc::carve(ws, B);
   tc::Finalize fin;
-  fin.val = best_val;
-  fin.idx = best_idx;
-  fin.R_best = R_best;
-  fin.idx_offset = idx_offset;
-  if (world > 1) {
-    if (world > peer::kMaxPeers || pa->rank < 0 || pa->rank >= world || B > pa->cap_pairs || pa->cap_k < 1) return AHV_EINVAL;
-    for (int r = 0; r < world; ++r)
-      if (!pa->bufs[r]) return AHV_EINVAL;
-    fin.peers = *pa;
-  }
+  const int st = make_finalize(best_val, best_idx, R_best, idx_offset, B, pa, &fin);
+  if (st != AHV_OK) return st;
   return dispatch(vol_src, vol_dtype, f16_gather, vol_tgt, nullptr, R, r_per_pair, W1, W2, b2, base, scores, true,
-                  B, N, sc, fin, s);
+                  B, N, tc::carve(ws, B), fin, s);
+}
+
+// The same step for fp32 volumes with the fp32 gather's result, screened by the 16-bit gather (1.6x its rate):
+//   pass 1  the 16-bit gather scores every hypothesis into `s16` [B,N]; its arg-max keys give each pair's screened
+//           maximum m_b (prologue: target features, key clear);
+//   select  per pair the contenders {n : s16[b,n] >= m_b - 2 tau} (at most kScreenCap) and kScreenProbes strided
+//           probes; their rotations are copied into s16's space as [B][kScreenList][9] per-pair rotation sets;
+//   pass 2  the fp32 gather scores the lists;
+//   guard   the list's fp32 arg-max key (original index: ties -> lowest) replaces the pair's screened key; the pair is
+//           flagged when some |s32 - s16| on its list exceeds tau / 4, or it had no or too many contenders;
+//   pass 3  the fp32 gather scores every hypothesis of the flagged pairs (their number is read on the device: zero
+//           items when none), publishes into the same keys, and its last CTA decodes them or runs the exchange.
+// A hypothesis's score depends on (pair, rotation) alone, not on the tile or CTA it is scored in, so the fp32 winner is
+// the single pass's bit for bit whenever it is on its pair's list - which holds when every 16-bit score lies within
+// tau of its fp32 score: then s16[w] >= s32[w] - tau >= s32[n*] - tau >= m_b - 2 tau (n* the screened arg-max).
+// `s16` must hold B*N floats and at least kScreenList*40 bytes per pair; `lists` ScreenLists::bytes(B).  No host
+// synchronisation: graph-capturable.
+int launch_verify_tc_screened(const float* vol_src, const float* vol_tgt, const float* R, int r_per_pair, const float* W1,
+                              const float* W2, const float* b2, const float* base, float* best_val, int64_t* best_idx,
+                              float* R_best, int64_t idx_offset, int B, int64_t N, void* ws, size_t ws_bytes, float* s16,
+                              void* lists, cudaStream_t s, const peer::Args* pa) {
+  if (ws_bytes < tc::scratch_bytes(B)) return AHV_EWORKSPACE;
+  tc::Finalize fin;
+  int st = make_finalize(best_val, best_idx, R_best, idx_offset, B, pa, &fin);
+  if (st != AHV_OK) return st;
+  const tc::Scratch sc = tc::carve(ws, B);
+  const ScreenLists L(lists, B);
+  float* R_list = s16;                                          // [B][kScreenList][9], after the selection
+  float* s32 = s16 + (size_t)B * kScreenList * 9;               // [B][kScreenList]
+  st = tc::launch_typed<float, true>(vol_src, vol_tgt, nullptr, R, r_per_pair, W1, W2, b2, base, s16, true, B, N, sc,
+                                     tc::Finalize{}, s);
+  if (st != AHV_OK) return st;
+  st = launch_screen_select(s16, sc.best_keys, B, N, R, r_per_pair, L, R_list, s);
+  if (st != AHV_OK) return st;
+  st = tc::launch_typed<float, false>(vol_src, nullptr, sc.tgt_feat, R_list, 1, W1, W2, b2, base, s32, false, B, kScreenList,
+                                      sc, tc::Finalize{}, s);
+  if (st != AHV_OK) return st;
+  st = launch_screen_guard(s32, L, B, sc.best_keys, s);
+  if (st != AHV_OK) return st;
+  return tc::launch_typed<float, false>(vol_src, nullptr, sc.tgt_feat, R, r_per_pair, W1, W2, b2, base, nullptr, true, B, N,
+                                        sc, fin, s, L.flagged);
 }
 
 }  // namespace ahv

@@ -45,13 +45,16 @@ score_tc_ts_kernel(const __grid_constant__ CUtensorMap vol_map, const float* __r
                    const float* __restrict__ R, int r_per_pair, const float* __restrict__ b2,
                    const float* __restrict__ base, const float* __restrict__ W1,
                    const float* __restrict__ W2, float* __restrict__ scores,
-                   u64* __restrict__ best_keys, int B, int64_t N, Finalize fin, int late_ctas) {
+                   u64* __restrict__ best_keys, int B, int64_t N, Finalize fin, int late_ctas,
+                   const int* __restrict__ pair_list) {
   extern __shared__ __align__(128) unsigned char smem[];
   using M = MapTS;
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;  // provably warp-uniform
   Work work;
   {
-    const int64_t total = (int64_t)B * N;
+    // pair_list = [count, pair...]: score the `count` listed pairs only (their number is known on the device alone)
+    const int64_t total = (pair_list ? (int64_t)min(__ldg(pair_list), B) : (int64_t)B) * N;
+    if (pair_list) work.map = pair_list + 1;
     // Contiguous, near-equal item ranges.  When the target-feature prologue of a SMALL batch precedes this kernel
     // (programmatic dependent launch), the last `late_ctas` CTAs - the ones that get the SMs the prologue's CTAs
     // occupy - start about one tile time late (in-kernel timeline: +2.4 us at B = 1); they are given one tile
@@ -65,7 +68,10 @@ score_tc_ts_kernel(const __grid_constant__ CUtensorMap vol_map, const float* __r
     work.hi = cut((int64_t)blockIdx.x + 1);
     work.N = N;
   }
-  if (work.lo >= work.hi) return;
+  if (work.lo >= work.hi) {  // no items: the fused selection still needs this CTA's ticket
+    if (best_keys && fin.val && warp == 0) finalize_ticket(fin, best_keys, R, r_per_pair, N, B, lane);
+    return;
+  }
   if (threadIdx.x == 0) AHV_TL(0);
 
   float* vol = reinterpret_cast<float*>(smem + M::off_vol);
@@ -95,7 +101,7 @@ score_tc_ts_kernel(const __grid_constant__ CUtensorMap vol_map, const float* __r
     const uint32_t bar = bar0 + (kVolFull + (vol_req & 1)) * 8;
     if (elect_one()) {
       mbar_arrive_expect_tx(bar, kC * kVox * (uint32_t)sizeof(T));
-      tma_load_3d(s_base + M::off_a + stage_buf * M::tile_bytes, &vol_map, bar, 0, 0, pair * kC);
+      tma_load_3d(s_base + M::off_a + stage_buf * M::tile_bytes, &vol_map, bar, 0, 0, work.pair(pair) * kC);
     }
     ++vol_req;
   };
@@ -183,7 +189,7 @@ score_tc_ts_kernel(const __grid_constant__ CUtensorMap vol_map, const float* __r
     // aligned 16-byte loads of the row's 48-byte window + selects: 13 % (fp32) / 30 % (16-bit) slower still.
     float Rn[9];
     auto fetch_R = [&](int fb, uint32_t fn) {
-      const float* Rg = R + (r_per_pair ? ((size_t)fb * N + fn) : (size_t)fn) * 9;
+      const float* Rg = R + (r_per_pair ? ((size_t)work.pair(fb) * N + fn) : (size_t)fn) * 9;
 #pragma unroll
       for (int e = 0; e < 9; ++e) Rn[e] = __ldg(Rg + e);
     };

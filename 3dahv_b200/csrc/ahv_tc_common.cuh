@@ -124,7 +124,43 @@ __device__ __forceinline__ void peer_exchange_and_merge(const Finalize& fin, con
 
 struct Work {  // contiguous range of (pair, hypothesis) items of this CTA
   int64_t lo, hi, N;
+  // pairs of the item range are the listed ones when set (the fallback pass of the screened arg-max scores only the
+  // pairs it flagged): item pair b is pair map[b].  The ring of pair scales stays indexed by the item pair.
+  const int* map = nullptr;
+  __device__ __forceinline__ int pair(int b) const { return map ? __ldg(map + b) : b; }
 };
+
+// Ticket of a CTA whose keys are published: the last CTA of the grid decodes the arg-max keys into (score, index,
+// rotation), or exchanges and merges them with the peers' when the set is sharded.  One warp.
+__device__ __forceinline__ void finalize_ticket(const Finalize& fin, const u64* best_keys, const float* R, int r_per_pair,
+                                                int64_t N, int B, int lane) {
+  __syncwarp();
+  unsigned last = 0;
+  if (lane == 0) {
+    __threadfence();  // this CTA's keys before its ticket
+    last = atomicAdd(fin.counter, 1u) == gridDim.x - 1;
+  }
+  last = __shfl_sync(0xffffffffu, last, 0);
+  if (last && fin.peers.world > 1) {
+    __threadfence();
+    peer_exchange_and_merge(fin, best_keys, R, r_per_pair, N, B, lane);
+    if (lane == 0) *fin.counter = 0u;
+  } else if (last) {  // every other CTA has published its keys
+    __threadfence();
+    for (int b = lane; b < B; b += 32) {
+      const u64 key = __ldcg(best_keys + b);
+      const uint32_t n = key_index(key);
+      fin.val[b] = key_score(key);
+      fin.idx[b] = (int64_t)n + fin.idx_offset;
+      if (fin.R_best) {
+        const float* src = R + ((r_per_pair ? (size_t)b * N : 0) + (size_t)n) * 9;
+#pragma unroll
+        for (int e = 0; e < 9; ++e) fin.R_best[b * 9 + e] = __ldg(src + e);
+      }
+    }
+    if (lane == 0) *fin.counter = 0u;
+  }
+}
 
 // tile = two consecutive hypotheses of one pair; advance() returns false when exhausted.  All per-tile
 // state is 32-bit (N <= 2^31-1 and the CTA's share of B*N < 2^32 are checked on the host): the iterator
@@ -375,12 +411,13 @@ __device__ __forceinline__ void epilogue_role(const Work& work, int s, int lane,
       const float* pp = partial + (gb * 2 + lane) * 4;
       const float tot = ((pp[0] + pp[1]) + pp[2]) + pp[3];  // fixed order: deterministic
       const float sc = tot * (1.0f / 64.0f);                // .mean(dim=-1)
-      if (scores) scores[(size_t)pb * N + pn0 + lane] = sc;
+      const int rb = work.pair(pb);
+      if (scores) scores[(size_t)rb * N + pn0 + lane] = sc;
       if (best_keys) {
         const u64 key = make_key(sc, (uint32_t)(pn0 + lane));
-        if (pb != key_b) {
+        if (rb != key_b) {
           if (key_b >= 0) atomicMax(best_keys + key_b, key_best);
-          key_b = pb;
+          key_b = rb;
           key_best = key;
         } else if (key > key_best) {
           key_best = key;
@@ -428,7 +465,7 @@ __device__ __forceinline__ void epilogue_role(const Work& work, int s, int lane,
         if (s == 0 && lane == 0) fin.pair_inv_out[cur_b] = inv_pair * ws.w1;
       }
 #pragma unroll
-      for (int o = 0; o < kO; ++o) tg[o] = __ldg(tgt_feat + ((size_t)cur_b * kO + o) * kP + pos);
+      for (int o = 0; o < kO; ++o) tg[o] = __ldg(tgt_feat + ((size_t)work.pair(cur_b) * kO + o) * kP + pos);
     }
     prev_b = it.b; prev_n0 = it.n0; prev_cnt = it.cnt; prev_inv = inv_s;
     ++g;
@@ -436,34 +473,7 @@ __device__ __forceinline__ void epilogue_role(const Work& work, int s, int lane,
   phase_b(g - 1, prev_b, prev_n0, prev_cnt, prev_inv);
   if (s == 0 && lane == 0) AHV_TL(9);
   if (best_keys && key_b >= 0) atomicMax(best_keys + key_b, key_best);
-  if (best_keys && fin.val && s == 0) {
-    __syncwarp();
-    unsigned last = 0;
-    if (lane == 0) {
-      __threadfence();  // this CTA's keys before its ticket
-      last = atomicAdd(fin.counter, 1u) == gridDim.x - 1;
-    }
-    last = __shfl_sync(0xffffffffu, last, 0);
-    if (last && fin.peers.world > 1) {
-      __threadfence();
-      peer_exchange_and_merge(fin, best_keys, R, r_per_pair, N, B, lane);
-      if (lane == 0) *fin.counter = 0u;
-    } else if (last) {  // every other CTA has published its keys
-      __threadfence();
-      for (int b = lane; b < B; b += 32) {
-        const u64 key = __ldcg(best_keys + b);
-        const uint32_t n = key_index(key);
-        fin.val[b] = key_score(key);
-        fin.idx[b] = (int64_t)n + fin.idx_offset;
-        if (fin.R_best) {
-          const float* src = R + ((r_per_pair ? (size_t)b * N : 0) + (size_t)n) * 9;
-#pragma unroll
-          for (int e = 0; e < 9; ++e) fin.R_best[b * 9 + e] = __ldg(src + e);
-        }
-      }
-      if (lane == 0) *fin.counter = 0u;
-    }
-  }
+  if (best_keys && fin.val && s == 0) finalize_ticket(fin, best_keys, R, r_per_pair, N, B, lane);
 }
 
 }  // namespace tc

@@ -96,6 +96,103 @@ __global__ void gather_rotations_kernel(const float* __restrict__ R, int r_per_p
   out[t] = v;
 }
 
+// ---- screened arg-max of ahv_verify (see launch_verify_tc_screened in ahv_score_tc.cu) --------------------------
+// select: one CTA per pair collects the contenders {n : s16[b,n] >= m_b - 2 tau}, m_b = the pair's screened maximum
+// (its arg-max key), in no particular order; pads to kScreenCap with the first; appends the strided probes.
+constexpr int kSelectThreads = 512;
+__global__ void __launch_bounds__(kSelectThreads)
+screen_select_kernel(const float* __restrict__ s16, const u64* __restrict__ keys, int N, ScreenLists L) {
+  __shared__ int cnt;
+  __shared__ int sidx[kScreenCap];
+  __shared__ float sval[kScreenCap];
+  const int b = blockIdx.x, t = threadIdx.x;
+  if (t == 0) {
+    cnt = 0;
+    if (b == 0) L.flagged[0] = 0;
+  }
+  __syncthreads();
+  const float* row = s16 + (size_t)b * N;
+  const float lo = key_score(keys[b]) - 2.0f * kScreenTau;  // NaN maximum: no contender, the pair is flagged
+#pragma unroll 8
+  for (int n = t; n < N; n += kSelectThreads) {
+    const float v = row[n];
+    if (v >= lo) {
+      const int p = atomicAdd(&cnt, 1);
+      if (p < kScreenCap) { sidx[p] = n; sval[p] = v; }
+    }
+  }
+  __syncthreads();
+  const int c = min(cnt, kScreenCap);
+  for (int i = t; i < kScreenList; i += kSelectThreads) {
+    int n;
+    float v;
+    if (i < c) {
+      n = sidx[i]; v = sval[i];
+    } else if (i < kScreenCap && c > 0) {
+      n = sidx[0]; v = sval[0];
+    } else {
+      n = (int)((int64_t)(i < kScreenCap ? 0 : i - kScreenCap) * N / kScreenProbes);
+      v = row[n];
+    }
+    L.idx[(size_t)b * kScreenList + i] = n;
+    L.s16[(size_t)b * kScreenList + i] = v;
+  }
+  if (t == 0) L.count[b] = cnt;
+}
+
+// the rotations of every list entry, [B][kScreenList][9]: the fp32 pass scores them as per-pair rotation sets
+__global__ void __launch_bounds__(kScreenList)
+screen_gather_kernel(const float* __restrict__ R, int r_per_pair, int64_t N, ScreenLists L, float* __restrict__ R_list) {
+  const size_t at = (size_t)blockIdx.x * kScreenList + threadIdx.x;
+  const float* src = R + ((r_per_pair ? (size_t)blockIdx.x * N : 0) + (size_t)L.idx[at]) * 9;
+#pragma unroll
+  for (int e = 0; e < 9; ++e) R_list[at * 9 + e] = __ldg(src + e);
+}
+
+// guard: the list's fp32 arg-max key (original indices) replaces the pair's screened key; the pair is flagged for the
+// exact pass when a realised |s32 - s16| on its list exceeds tau / 4 (or is NaN), or it had no or too many contenders
+__global__ void __launch_bounds__(kScreenList)
+screen_guard_kernel(const float* __restrict__ s32, ScreenLists L, u64* __restrict__ keys) {
+  __shared__ u64 wkey[kScreenList / 32];
+  __shared__ float werr[kScreenList / 32];
+  const int b = blockIdx.x, t = threadIdx.x, lane = t & 31;
+  const size_t at = (size_t)b * kScreenList + t;
+  const float v = s32[at];
+  float e = fabsf(v - L.s16[at]);
+  const bool bad = !(e <= 0.25f * kScreenTau);
+  u64 key = make_key(v, (uint32_t)L.idx[at]);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    key = umax64(key, __shfl_xor_sync(0xffffffffu, key, o));
+    e = fmaxf(e, __shfl_xor_sync(0xffffffffu, e, o));
+  }
+  if (lane == 0) { wkey[t >> 5] = key; werr[t >> 5] = e; }
+  const int any_bad = __syncthreads_or(bad);
+  if (t == 0) {
+    for (int w = 1; w < kScreenList / 32; ++w) { key = umax64(key, wkey[w]); e = fmaxf(e, werr[w]); }
+    keys[b] = key;
+    L.err[b] = e;  // fmaxf skips NaN errors; they flag the pair all the same
+    const int c = L.count[b];
+    if (any_bad || c < 1 || c > kScreenCap) L.flagged[1 + atomicAdd(L.flagged, 1)] = b;
+  }
+}
+
+int launch_screen_select(const float* s16, const u64* keys, int B, int64_t N, const float* R, int r_per_pair,
+                         const ScreenLists& L, float* R_list, cudaStream_t s) {
+  screen_select_kernel<<<B, kSelectThreads, 0, s>>>(s16, keys, (int)N, L);
+  AHV_CUDA_OK(cudaGetLastError());
+  // R_list overwrites s16: launched after every pair's selection
+  screen_gather_kernel<<<B, kScreenList, 0, s>>>(R, r_per_pair, N, L, R_list);
+  AHV_CUDA_OK(cudaGetLastError());
+  return AHV_OK;
+}
+
+int launch_screen_guard(const float* s32, const ScreenLists& L, int B, u64* keys, cudaStream_t s) {
+  screen_guard_kernel<<<B, kScreenList, 0, s>>>(s32, L, keys);
+  AHV_CUDA_OK(cudaGetLastError());
+  return AHV_OK;
+}
+
 static int slices_for(int64_t N) {
   int64_t s = N / 4096;
   if (s < 1) s = 1;

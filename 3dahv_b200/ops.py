@@ -5,6 +5,8 @@ path happens inside lib3dahv_b200.so.
 """
 from __future__ import annotations
 
+import ctypes
+
 import torch
 import torch.nn.functional as F
 
@@ -377,6 +379,23 @@ def verify(vol_src, vol_tgt, R, W1, W2, b2, k: int = 1, idx_offset: int = 0, mat
           b2.data_ptr(), base_coords(dev).data_ptr(), scores.data_ptr() if scores is not None else None, val.data_ptr(),
           idx.data_ptr(), Rb.data_ptr() if Rb is not None else None, k, idx_offset, B, N, math, workspace.data_ptr(), ws_bytes)
     return scores, val, idx, Rb
+
+
+def verify_screen_stats(workspace: torch.Tensor | None, B: int, N: int):
+    """What the last screened `verify` (k = 1, fp32 volumes, MATH_TC, no scores) over `workspace` found: None when a
+    call of that shape takes the single pass, else (number of pairs that fell back to the exact pass, contenders per
+    pair [B] int32, largest |fp32 - 16-bit| score difference on each pair's list [B] fp32).  Synchronises."""
+    lib = _lib.lib()
+    is_screened = ctypes.c_int(0)
+    _lib.check(lib.ahv_verify_screen_stats(None, B, N, ctypes.byref(is_screened), None, None, None), "ahv_verify_screen_stats")
+    if not is_screened.value:
+        return None
+    flagged = ctypes.c_int(0)
+    count = (ctypes.c_int * B)()
+    err = (ctypes.c_float * B)()
+    _lib.check(lib.ahv_verify_screen_stats(workspace.data_ptr(), B, N, ctypes.byref(is_screened), ctypes.byref(flagged),
+                                           count, err), "ahv_verify_screen_stats")
+    return flagged.value, torch.tensor(list(count), dtype=torch.int32), torch.tensor(list(err), dtype=torch.float32)
 
 
 def refine(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, m: int = 64, max_angle_deg: float = 5.0, seed: int = 0,

@@ -242,11 +242,28 @@ AHV_API int ahv_score(const void* vol_src, int vol_dtype, const float* tgt_feat,
  * is two launches — the target-feature prologue, and the fused scoring kernel (launched programmatically
  * dependent on it; packs the weights and derives the per-pair scales itself) with the arg-max folded
  * into its epilogue and the winners decoded by its last CTA.
+ * Screened form: with fp32 volumes, AHV_MATH_TC, k == 1, scores == NULL and B*N >= 2^18 (and N >= about 37 000, so
+ * that its lists fit the workspace ahv_workspace_bytes sizes) the step is seven launches: the 16-bit gather
+ * (AHV_MATH_TC_F16GATHER's kernel, 1.6x the fp32 gather's rate) scores every hypothesis; per pair, the hypotheses
+ * within 2 tau (tau = 2e-3 in score units) of its best 16-bit score, at most 224, and 32 strided probes are re-scored by
+ * the fp32 gather; a pair whose realised |fp32 - 16-bit| difference on that list exceeds tau / 4, or which has more
+ * than 224 contenders, is scored again in full by the fp32 gather (the number of such pairs is read on the device:
+ * no host synchronisation, CUDA-graph capturable).  The result equals the single pass's bit for bit whenever every
+ * hypothesis's 16-bit score lies within tau of its fp32 score; that is checked on every call on each pair's list,
+ * with the per-pair fallback behind it - a checked margin, not a proof.  Every other call is the single pass.
  * scores [B,N] or NULL; topk_val/topk_idx [B,k]; R_best [B,k,3,3] or NULL. */
 AHV_API int ahv_verify(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
                        const float* W1, const float* W2, const float* b2, const float* base, float* scores,
                        float* topk_val, int64_t* topk_idx, float* R_best, int k, int64_t idx_offset, int B,
                        int64_t N, int math_mode, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Diagnostics of the screened form of ahv_verify (and ahv_verify_sharded, per rank with the rank's N): *is_screened =
+ * whether a call with (B, N), fp32 volumes, AHV_MATH_TC, k == 1 and no scores takes it.  If so and any of the other
+ * outputs is set, reads what the last such call over `workspace` left there (synchronising copies):
+ * flagged_pairs = pairs scored again in full, contenders [B] = hypotheses within 2 tau of each pair's best 16-bit
+ * score (more than 224: overflow), max_err [B] = the largest |fp32 - 16-bit| score difference on each pair's list. */
+AHV_API int ahv_verify_screen_stats(const void* workspace, int B, int64_t N, int* is_screened, int* flagged_pairs,
+                                    int* contenders, float* max_err);
 
 /* Two-pass selection in one call (extension, BASELINE config 4 "dense SO(3) grid with top-k refinement pass";
  * the reference stops at torch.max over its random set, test_linemod.py:62-63): ahv_verify over the N
