@@ -120,43 +120,13 @@ __device__ __forceinline__ float key_score(u64 key) {
 }
 __device__ __forceinline__ uint32_t key_index(u64 key) { return 0xFFFFFFFFu - (uint32_t)key; }
 
-// Ascending sort of a[0 .. kM) in registers (kM <= kN, kN a power of two; a[kM .. kN) hold 0xffffffff): Batcher's
-// odd-even merge network for kN inputs, fully unrolled, without the comparators that touch a place >= kM.  Every
-// comparator puts the smaller value at the lower place, so those places keep the largest value and their comparators
-// are no-ops.  19, 42 and 63 comparators for (8, 8), (16, 12) and (16, 16) (each checked on all 0-1 inputs).
-template <int kN, int kM>
-__device__ __forceinline__ void oddeven_sort(uint32_t* a) {
-#pragma unroll
-  for (int p = 1; p < kN; p <<= 1)
-#pragma unroll
-    for (int k = p; k >= 1; k >>= 1)
-#pragma unroll
-      for (int x = 0; x < kN; ++x)   // comparator (x, x + k): x = j + i, j = k % p (mod 2k), i < k, same 2p-block
-        if (x + k < kM && x >= k % p && (x - k % p) % (2 * k) < k && x / (2 * p) == (x + k) / (2 * p)) {
-          const uint32_t lo = min(a[x], a[x + k]);
-          a[x + k] = max(a[x], a[x + k]);
-          a[x] = lo;
-        }
+// SM count of the current device, 0 when it cannot be read
+inline int sm_count() {
+  int dev = 0, sms = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) return 0;
+  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
+  return sms;
 }
-// the n <= 16 register values of a warp whose largest count is nmax (warp-uniform)
-__device__ __forceinline__ void sort_row(uint32_t* a, int nmax) {
-  if (nmax <= 8) oddeven_sort<8, 8>(a);
-  else if (nmax <= 12) oddeven_sort<16, 12>(a);
-  else oddeven_sort<16, 16>(a);
-}
-
-// Insertion sort of one adjoint work list (offset of dX[vo], weight) by offset, which is unique per output voxel vo:
-// the deterministic backward sums every input voxel's contributions in this order, not in the order shared-memory
-// atomics handed out the places.  A rotation puts about 8 (at most ~12) entries on a voxel.
-__device__ __forceinline__ void sort_list(uint2* e, int n) {
-  for (int i = 1; i < n; ++i) {
-    const uint2 x = e[i];
-    int k = i;
-    for (; k > 0 && e[k - 1].x > x.x; --k) e[k] = e[k - 1];
-    e[k] = x;
-  }
-}
-
 
 namespace peer { struct Args; }  // ahv_peer.cuh
 
@@ -172,15 +142,18 @@ int launch_rotate_volume_bwd(const float* grad_out, int per_rot, const float* R,
                              float* grad_vol, int64_t n, cudaStream_t s);
 int launch_rotate_volume_grad_R(const float* vol, int per_rot, const float* R, const float* base, const float* grad_out,
                                 float* grad_R, int64_t n, cudaStream_t s);
+// The fused backward kernels (ahv_score_bwd.cu, ahv_score_bwd_tc.cu) on `grid` CTAs, 0: one per SM (at most one per
+// item).  det: the deterministic instance, whose outputs are the workspace slots below (launch_score_bwd_det).
 int launch_score_bwd(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
                      const float* W1, const float* W2, const float* b2, const float* base,
                      const float* grad_scores, float* g_vol, float* g_tgt, float* g_W1, float* g_W2,
                      float* g_b2, int B, int64_t N, cudaStream_t s, const void* h1_saved = nullptr,
-                     const float* pair_inv = nullptr, float* g_R = nullptr);
+                     const float* pair_inv = nullptr, float* g_R = nullptr, unsigned grid = 0, bool det = false);
 int launch_score_bwd_tc(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
                         const float* W1, const float* W2, const float* b2, const float* base,
                         const float* grad_scores, const void* h1_saved, const float* pair_inv, float* g_vol,
-                        float* g_tgt, float* g_W1, float* g_W2, float* g_b2, int B, int64_t N, cudaStream_t s);
+                        float* g_tgt, float* g_W1, float* g_W2, float* g_b2, int B, int64_t N, cudaStream_t s,
+                        unsigned grid = 0, bool det = false);
 // Deterministic backward (ahv_score_backward_det).  The kernels store what the atomic instances add into global memory
 // in per-CTA workspace slots, and score_bwd_det_reduce adds the slots of every output element in increasing slot order.
 //   weight slot c (one per CTA, c < grid):   dW1 [32][384] | dW2 [32][32] | db2 [32]              kDetWSlot floats
@@ -204,10 +177,6 @@ int launch_score_bwd_det(const float* vol_src, const float* tgt_feat, const floa
                          const float* W1, const float* W2, const float* b2, const float* base, const float* grad_scores,
                          const void* h1_saved, const float* pair_inv, float* g_vol, float* g_tgt, float* g_W1,
                          float* g_W2, float* g_b2, float* g_R, int B, int64_t N, bool tc, float* ws, cudaStream_t s);
-int launch_score_bwd_tc_det(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
-                            const float* W1, const float* W2, const float* b2, const float* base,
-                            const float* grad_scores, const void* h1_saved, const float* pair_inv, float* ws_w,
-                            float* ws_seg, int B, int64_t N, unsigned grid, cudaStream_t s);
 int launch_score_tc_train(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair, const float* W1,
                           const float* W2, const float* b2, const float* base, float* scores, void* h1_out,
                           float* pair_inv_out, int B, int64_t N, void* ws, size_t ws_bytes, cudaStream_t s);

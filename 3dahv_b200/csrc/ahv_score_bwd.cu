@@ -24,7 +24,10 @@
 // ~130k cycles per hypothesis): every INPUT voxel gets the list of the (output voxel, weight) contributions that reach
 // it (counting sort over the <= 4096 contributions with integer shared-memory atomics and prefix sums), and every
 // thread walks the lists of its two input voxels - exactly the output voxels that touch them, whatever the matrix R
-// is - reading dX, which lies voxel-major with the channels innermost, as four LDS.128 per contribution.
+// is - reading dX, which lies voxel-major with the channels innermost, as four LDS.128 per contribution.  The work
+// list, the orders the deterministic form sums it in and the flushes of the gradients are shared with the tcgen05
+// backward (ahv_adjoint.cuh).
+#include "ahv_adjoint.cuh"
 #include "ahv_bwd_fp32.cuh"
 
 namespace ahv {
@@ -42,13 +45,6 @@ static_assert((kDxFloats + 2 * kVox * 8) <= 2 * kC * kRotC + kP * kH1Row, "dX an
 static_assert(2 * kVox * sizeof(int) <= sizeof(float) * kP * kH1Row, "counters fit the dH2 buffer");
 static_assert((2 * kVox + 9 * kThreads / 32) * sizeof(float) <= sizeof(float) * kP * kH1Row,
               "the rotation phase's partial sums fit behind the counters");
-
-// output voxel (z*64 + y*8 + x) a thread lists for the adjoint: lane bits -> x2 x1 y2 y1 z2, warp bits and j -> the rest
-__device__ __forceinline__ int adjoint_out_voxel(int t, int j) {
-  const int x = ((t & 3) << 1) | ((t >> 5) & 1), y = (((t >> 2) & 3) << 1) | ((t >> 6) & 1);
-  const int z = (((t >> 4) & 1) << 2) | (((t >> 7) & 1) << 1) | j;
-  return z * 64 + y * 8 + x;
-}
 
 // kEx (ahv_score_backward_ex): every gradient output may be NULL - its accumulation and, for g_vol / g_W1 / g_R, its
 // phase are skipped - and the rotation-gradient phase (dS/dR into g_R) is compiled in.  kEx = false is the plain
@@ -98,43 +94,14 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
 #pragma unroll
     for (int c = 0; c < kC; ++c) aV[j][c] = 0.0f;
 
-  auto flush_pair = [&](int b) {  // dT and dV of pair b leave the CTA
-    if constexpr (kDet) {   // the whole segment, zeros included, into slot blockIdx.x + b
-      const size_t slot = (size_t)(blockIdx.x + b) * kDetSegSlot;
-#pragma unroll
-      for (int oo = 0; oo < 8; ++oo) {
-        if (want_tgt) g_tgt[slot + (cg2 * 8 + oo) * kP + pos] = aT[oo];
-        aT[oo] = 0.0f;
-      }
-#pragma unroll
-      for (int j = 0; j < 2; ++j)
-#pragma unroll
-        for (int c = 0; c < kC; ++c) {
-          if (want_vol) g_vol[slot + c * kVox + t + 256 * j] = aV[j][c];
-          aV[j][c] = 0.0f;
-        }
-    } else {
-#pragma unroll
-    for (int oo = 0; oo < 8; ++oo) {
-      if (want_tgt && aT[oo] != 0.0f) atomicAdd(g_tgt + ((size_t)b * kO + cg2 * 8 + oo) * kP + pos, aT[oo]);
-      aT[oo] = 0.0f;
-    }
-#pragma unroll
-    for (int j = 0; j < 2; ++j)
-#pragma unroll
-      for (int c = 0; c < kC; ++c) {
-        if (want_vol && aV[j][c] != 0.0f) atomicAdd(g_vol + ((size_t)b * kC + c) * kVox + t + 256 * j, aV[j][c]);
-        aV[j][c] = 0.0f;
-      }
-    }
-  };
+  auto flush = [&](int b) { flush_pair<kDet>(g_tgt, g_vol, b, aT, aV, cg2, pos, want_tgt, want_vol); };
 
   int cur_b = -1;
   for (int64_t it = lo; it < hi; ++it) {
     const int b = (int)(it / N);
     const int64_t n = it - (int64_t)b * N;
     if (b != cur_b) {
-      if (cur_b >= 0) flush_pair(cur_b);
+      if (cur_b >= 0) flush(cur_b);
       __syncthreads();
       stage_volume<float>(sm.vol, vol_src + (size_t)b * kC * kVox);
 #pragma unroll
@@ -235,87 +202,38 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
     }
 
     // ---------------- dV_b += rotate^T(dX): adjoint of utils.py:113-131 as a gather ----------------
-    // Output voxel vo feeds the 8 input voxels of its tap, corner(vo) + {0,1}^3, with the forward's weights.  Turned round:
-    // every INPUT voxel gets the list of its (vo, weight) contributions - a counting sort over the <= 4096 contributions
-    // that land inside the volume (shared-memory integer atomics whose return value is the place in the list, prefix
-    // sums, 8-byte entries behind dX in the dead rotated-volume / dH1 buffers) - and the adjoint is one flat loop per
-    // input voxel: exactly the contributing voxels, no geometry test, valid for any matrix R, fp32 weights recomputed from
-    // the taps the forward gather recorded.
+    // Every INPUT voxel gets the list of its (output voxel, weight) contributions (build_exact_list, ahv_adjoint.cuh: 8-byte
+    // entries behind dX in the dead rotated-volume / dH1 buffers), and the adjoint is one flat loop per input voxel:
+    // exactly the contributing voxels, no geometry test, valid for any matrix R, fp32 weights recomputed from the taps
+    // the forward gather recorded.
     if (want_vol) {
       int* cnt = reinterpret_cast<int*>(bs.dh2);   // [512] contributions per input voxel
       int* start = cnt + kVox;                     // [512] exclusive prefix sum
       uint2* ent = reinterpret_cast<uint2*>(smem_raw + offsetof(BwdSmem, f) + offsetof(Fp32Smem, rotA) + sizeof(float) * kDxFloats);   // [<= 4096] (offset of dX[vo], weight), behind dX
-      cnt[t] = 0;
-      cnt[t + 256] = 0;
+      // sm.red is free outside volume staging: the scan's 8 warp totals
+      build_exact_list<kDxD, kDxH, kDxW>(bs.taps, cnt, start, ent, reinterpret_cast<int*>(sm.red));
       __syncthreads();
-      // the thread's two output voxels: two apart in x and y, four in z across the lanes of a warp, so that the taps of one
-      // warp's voxels rarely meet in the same counter
-      int tgt0[2];
-      uint32_t inside[2], rank[2][4];
-      float fx[2], fy[2], fz[2];
+      // acc[0..15] += w * dX[vo][0..15]: four LDS.128 per contribution
+      auto axpy = [&](float* acc, uint2 en) {
+        const float w = __uint_as_float(en.y);
+        const float* src = sm.rotA + en.x;
+#pragma unroll
+        for (int c4 = 0; c4 < 4; ++c4) {
+          const float4 x = *reinterpret_cast<const float4*>(src + 4 * c4);
+          acc[4 * c4] = fmaf(w, x.x, acc[4 * c4]); acc[4 * c4 + 1] = fmaf(w, x.y, acc[4 * c4 + 1]);
+          acc[4 * c4 + 2] = fmaf(w, x.z, acc[4 * c4 + 2]); acc[4 * c4 + 3] = fmaf(w, x.w, acc[4 * c4 + 3]);
+        }
+      };
 #pragma unroll
       for (int j = 0; j < 2; ++j) {
-        const int vo = adjoint_out_voxel(t, j);
-        const float4 tp = bs.taps[vo];
-        const int line = __float_as_int(tp.x);   // ((z0+1)*10 + (y0+1))*10 + (x0+1), corner in [-1, 7]^3
-        const int zl = line / (kHalo * kHalo), rl = line - zl * (kHalo * kHalo), yl = rl / kHalo, xl = rl - yl * kHalo;
-        const int x0 = xl - 1, y0 = yl - 1, z0 = zl - 1;
-        fx[j] = tp.y; fy[j] = tp.z; fz[j] = tp.w;
-        tgt0[j] = z0 * 64 + y0 * 8 + x0;
-        uint32_t m = 0;
-        rank[j][0] = rank[j][1] = rank[j][2] = rank[j][3] = 0;
-#pragma unroll
-        for (int dlt = 0; dlt < 8; ++dlt) {
-          const int x = x0 + (dlt & 1), y = y0 + ((dlt >> 1) & 1), z = z0 + (dlt >> 2);
-          if ((unsigned)x < 8u && (unsigned)y < 8u && (unsigned)z < 8u) {
-            m |= 1u << dlt;   // the atomic's return value is this contribution's place in its list (<= 511: 16 bits)
-            rank[j][dlt >> 1] |= (uint32_t)atomicAdd(&cnt[tgt0[j] + (dlt >> 2) * 64 + ((dlt >> 1) & 1) * 8 + (dlt & 1)], 1) << (16 * (dlt & 1));
-          }
-        }
-        inside[j] = m;
-      }
-      __syncthreads();
-      {  // exclusive scan of the 512 counters: 2 per thread, warp scan, then the 8 warp totals
-        const int c0 = cnt[2 * t], c1 = cnt[2 * t + 1];
-        const int local = c0 + c1;
-        int incl = local;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const int up = __shfl_up_sync(0xffffffffu, incl, o);
-          if ((t & 31) >= o) incl += up;
-        }
-        int* wtot = reinterpret_cast<int*>(sm.red);          // 8 warp totals (sm.red is free outside volume staging)
-        if ((t & 31) == 31) wtot[t >> 5] = incl;
-        __syncthreads();
-        int basep = incl - local;
-        for (int w = 0; w < (t >> 5); ++w) basep += wtot[w];
-        start[2 * t] = basep;
-        start[2 * t + 1] = basep + c0;
-      }
-      __syncthreads();
-#pragma unroll
-      for (int j = 0; j < 2; ++j) {
-        const int vo = adjoint_out_voxel(t, j);
-        const uint32_t off = (uint32_t)((vo >> 6) * kDxD + ((vo >> 3) & 7) * kDxH + (vo & 7) * kDxW);
-#pragma unroll
-        for (int dlt = 0; dlt < 8; ++dlt)
-          if ((inside[j] >> dlt) & 1u) {
-            const int dx = dlt & 1, dy = (dlt >> 1) & 1, dz = dlt >> 2;
-            const float w = (dx ? fx[j] : 1.0f - fx[j]) * (dy ? fy[j] : 1.0f - fy[j]) * (dz ? fz[j] : 1.0f - fz[j]);
-            const int v = tgt0[j] + dz * 64 + dy * 8 + dx;
-            ent[start[v] + ((rank[j][dlt >> 1] >> (16 * (dlt & 1))) & 0xffffu)] = make_uint2(off, __float_as_uint(w));
-          }
-      }
-      __syncthreads();
-      if constexpr (kDet) {
-        // The atomics ranked each list in arrival order; it is summed in increasing dX offset instead.  Up to 16 entries
-        // (a rotation puts at most ~12 on a voxel) the keys (offset, place) are sorted in registers by a network and the
-        // entries read in that order; longer lists (matrices that crowd the samples) are sorted in place first.
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const int vi = t + 256 * j;
-          const int nn = cnt[vi];
-          uint2* e = ent + start[vi];
+        const int vi = t + 256 * j;
+        const int nn = cnt[vi];
+        uint2* e = ent + start[vi];
+        if constexpr (kDet) {
+          // The atomics ranked each list in arrival order; it is summed in increasing dX offset instead.  Up to 16
+          // entries (a rotation puts at most ~12 on a voxel) the keys (offset, place) are sorted in registers by a
+          // network and the entries read in that order; longer lists (matrices that crowd the samples) are sorted in
+          // place first.
           int nmax = nn;
 #pragma unroll
           for (int o = 16; o > 0; o >>= 1) nmax = max(nmax, __shfl_xor_sync(0xffffffffu, nmax, o));
@@ -327,59 +245,19 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
 #pragma unroll
             for (int i = 0; i < 16; ++i) {
               if (i >= nmax) break;   // warp-uniform
-              if (i < nn) {
-                const uint2 en = e[key[i] & 15u];
-                const float w = __uint_as_float(en.y);
-                const float* src = sm.rotA + en.x;
-#pragma unroll
-                for (int c4 = 0; c4 < 4; ++c4) {
-                  const float4 x = *reinterpret_cast<const float4*>(src + 4 * c4);
-                  aV[j][4 * c4] = fmaf(w, x.x, aV[j][4 * c4]); aV[j][4 * c4 + 1] = fmaf(w, x.y, aV[j][4 * c4 + 1]);
-                  aV[j][4 * c4 + 2] = fmaf(w, x.z, aV[j][4 * c4 + 2]); aV[j][4 * c4 + 3] = fmaf(w, x.w, aV[j][4 * c4 + 3]);
-                }
-              }
+              if (i < nn) axpy(aV[j], e[key[i] & 15u]);
             }
             continue;
           }
           sort_list(e, nn);
-#pragma unroll 2
-          for (int i = 0; i < nn; ++i) {
-            const uint2 en = e[i];
-            const float w = __uint_as_float(en.y);
-            const float* src = sm.rotA + en.x;
-#pragma unroll
-            for (int c4 = 0; c4 < 4; ++c4) {
-              const float4 x = *reinterpret_cast<const float4*>(src + 4 * c4);
-              aV[j][4 * c4] = fmaf(w, x.x, aV[j][4 * c4]); aV[j][4 * c4 + 1] = fmaf(w, x.y, aV[j][4 * c4 + 1]);
-              aV[j][4 * c4 + 2] = fmaf(w, x.z, aV[j][4 * c4 + 2]); aV[j][4 * c4 + 3] = fmaf(w, x.w, aV[j][4 * c4 + 3]);
-            }
-          }
         }
-      } else {
-#pragma unroll
-      for (int j = 0; j < 2; ++j) {
-        const int vi = t + 256 * j;
-        const int nn = cnt[vi];
-        const uint2* e = ent + start[vi];
-#pragma unroll 2
-        for (int i = 0; i < nn; ++i) {
-          const uint2 en = e[i];
-          const float w = __uint_as_float(en.y);
-          const float* src = sm.rotA + en.x;
-#pragma unroll
-          for (int c4 = 0; c4 < 4; ++c4) {
-            const float4 x = *reinterpret_cast<const float4*>(src + 4 * c4);
-            aV[j][4 * c4] = fmaf(w, x.x, aV[j][4 * c4]); aV[j][4 * c4 + 1] = fmaf(w, x.y, aV[j][4 * c4 + 1]);
-            aV[j][4 * c4 + 2] = fmaf(w, x.z, aV[j][4 * c4 + 2]); aV[j][4 * c4 + 3] = fmaf(w, x.w, aV[j][4 * c4 + 3]);
-          }
-        }
-      }
+        walk_list(e, nn, [&](uint2 en) { axpy(aV[j], en); });
       }
     }
     __syncthreads();  // dX, the work list and the taps are re-used by the next hypothesis
   }
-  flush_pair(cur_b);
-  // weight gradients: one atomic per accumulator and CTA
+  flush(cur_b);
+  // weight gradients: one atomic per accumulator and CTA (kDet: one store into the CTA's weight slot)
   {
     const int cg = t & 15, c = t >> 4;
 #pragma unroll
@@ -387,35 +265,16 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
 #pragma unroll
       for (int kk = 0; kk < 8; ++kk) {
         const int k = view * 128 + c * 8 + kk;
-        if constexpr (kDet) {
-          if (want_W1) {
-            g_W1[(size_t)blockIdx.x * kDetWSlot + (2 * cg) * kK + k] = aW1[view][kk][0];
-            g_W1[(size_t)blockIdx.x * kDetWSlot + (2 * cg + 1) * kK + k] = aW1[view][kk][1];
-          }
-        } else if (want_W1) {
-          atomicAdd(g_W1 + (2 * cg) * kK + k, aW1[view][kk][0]);
-          atomicAdd(g_W1 + (2 * cg + 1) * kK + k, aW1[view][kk][1]);
+        if (want_W1) {
+          flush_weight<kDet>(g_W1 + (2 * cg) * kK + k, aW1[view][kk][0]);
+          flush_weight<kDet>(g_W1 + (2 * cg + 1) * kK + k, aW1[view][kk][1]);
         }
       }
     const int o = t >> 3, i0 = (t & 7) * 4;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      if constexpr (kDet) {
-        if (want_W2) g_W2[(size_t)blockIdx.x * kDetWSlot + o * kO + i0 + i] = aW2[i];
-      } else if (want_W2) atomicAdd(g_W2 + o * kO + i0 + i, aW2[i]);
-    }
-    // db2: sum over the 64 positions inside the CTA first (threads with equal cg2 = t & 3)
-    __syncthreads();
-    float* red = sm.h1s;  // [4 cg2][8 oo][64 pos]
-#pragma unroll
-    for (int oo = 0; oo < 8; ++oo) red[(cg2 * 8 + oo) * kP + pos] = ab2[oo];
-    __syncthreads();
-    if (want_b2 && t < kO) {
-      float s = 0.0f;
-      for (int p = 0; p < kP; ++p) s += red[t * kP + p];
-      if constexpr (kDet) g_b2[(size_t)blockIdx.x * kDetWSlot + t] = s;
-      else atomicAdd(g_b2 + t, s);
-    }
+    for (int i = 0; i < 4; ++i)
+      if (want_W2) flush_weight<kDet>(g_W2 + o * kO + i0 + i, aW2[i]);
+    flush_b2<kDet>(sm.h1s, ab2, cg2, pos, g_b2, want_b2);   // sm.h1s: [4 cg2][8 oo][64 pos]
   }
 }
 
@@ -423,24 +282,21 @@ int launch_score_bwd(const float* vol_src, const float* tgt_feat, const float* R
                      const float* W1, const float* W2, const float* b2, const float* base,
                      const float* grad_scores, float* g_vol, float* g_tgt, float* g_W1, float* g_W2,
                      float* g_b2, int B, int64_t N, cudaStream_t s, const void* h1_saved, const float* pair_inv,
-                     float* g_R) {
+                     float* g_R, unsigned grid, bool det) {
   const int64_t total = (int64_t)B * N;
   if (total == 0) return AHV_OK;
-  int dev = 0, sms = 0;
-  AHV_CUDA_OK(cudaGetDevice(&dev));
-  AHV_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  const unsigned grid = (unsigned)(total < sms ? total : sms);
-  const size_t smem = sizeof(BwdSmem);
-  const __half* h1 = static_cast<const __half*>(h1_saved);
-  if (g_R || !g_vol || !g_tgt || !g_W1 || !g_W2 || !g_b2) {
-    AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    score_bwd_kernel<true, false><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
-                                                        g_vol, g_tgt, g_W1, g_W2, g_b2, B, N, h1, pair_inv, g_R);
-  } else {
-    AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    score_bwd_kernel<false, false><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
-                                                         g_vol, g_tgt, g_W1, g_W2, g_b2, B, N, h1, pair_inv, nullptr);
+  if (grid == 0) {
+    const int sms = sm_count();
+    if (sms <= 0) return AHV_ECUDA;
+    grid = (unsigned)(total < sms ? total : sms);
   }
+  const bool ex = g_R || !g_vol || !g_tgt || !g_W1 || !g_W2 || !g_b2;
+  const auto kernel = ex ? (det ? score_bwd_kernel<true, true> : score_bwd_kernel<true, false>)
+                         : (det ? score_bwd_kernel<false, true> : score_bwd_kernel<false, false>);
+  const size_t smem = sizeof(BwdSmem);
+  AHV_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores, g_vol, g_tgt,
+                                      g_W1, g_W2, g_b2, B, N, static_cast<const __half*>(h1_saved), pair_inv, g_R);
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }
@@ -500,42 +356,24 @@ int launch_score_bwd_det(const float* vol_src, const float* tgt_feat, const floa
                          float* g_W2, float* g_b2, float* g_R, int B, int64_t N, bool tc, float* ws, cudaStream_t s) {
   const int64_t total = (int64_t)B * N;
   if (total == 0) return AHV_OK;
-  int dev = 0, sms = 0;
-  AHV_CUDA_OK(cudaGetDevice(&dev));
-  AHV_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  const int sms = sm_count();
+  if (sms <= 0) return AHV_ECUDA;
   const int grid = (int)std::min<int64_t>(total, std::min(sms, kDetGridCap));
   const bool shared_R = g_R && !r_per_pair;
   const DetBwdWs w(B, N, shared_R);
-  float* ws_w = ws;
-  float* ws_seg = ws + w.seg;
-  if (tc) {
-    const int st = launch_score_bwd_tc_det(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores, h1_saved,
-                                           pair_inv, ws_w, ws_seg, B, N, (unsigned)grid, s);
-    if (st != AHV_OK) return st;
-  } else {
-    // the kernel's outputs are the workspace slots (NULL where the caller's output is NULL); a per-pair R's gradient
-    // has one writer per element and goes straight to the caller's buffer
-    float* k_vol = g_vol ? ws_seg : nullptr;
-    float* k_tgt = g_tgt ? ws_seg + kC * kVox : nullptr;
-    float* k_W1 = g_W1 ? ws_w : nullptr;
-    float* k_W2 = g_W2 ? ws_w + kO * kK : nullptr;
-    float* k_b2 = g_b2 ? ws_w + kO * kK + kO * kO : nullptr;
-    float* k_R = g_R ? (r_per_pair ? g_R : ws + w.rot) : nullptr;
-    const size_t smem = sizeof(BwdSmem);
-    const __half* h1 = static_cast<const __half*>(h1_saved);
-    if (g_R || !g_vol || !g_tgt || !g_W1 || !g_W2 || !g_b2) {
-      AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      score_bwd_kernel<true, true><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base,
-                                                                grad_scores, k_vol, k_tgt, k_W1, k_W2, k_b2, B, N, h1,
-                                                                pair_inv, k_R);
-    } else {
-      AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      score_bwd_kernel<false, true><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base,
-                                                                 grad_scores, k_vol, k_tgt, k_W1, k_W2, k_b2, B, N, h1,
-                                                                 pair_inv, nullptr);
-    }
-    AHV_CUDA_OK(cudaGetLastError());
-  }
+  // the kernel's outputs are the workspace slots (NULL where the caller's output is NULL); a per-pair R's gradient
+  // has one writer per element and goes straight to the caller's buffer
+  float* k_vol = g_vol ? ws + w.seg : nullptr;
+  float* k_tgt = g_tgt ? ws + w.seg + kC * kVox : nullptr;
+  float* k_W1 = g_W1 ? ws : nullptr;
+  float* k_W2 = g_W2 ? ws + kO * kK : nullptr;
+  float* k_b2 = g_b2 ? ws + kO * kK + kO * kO : nullptr;
+  float* k_R = g_R ? (r_per_pair ? g_R : ws + w.rot) : nullptr;
+  const int st = tc ? launch_score_bwd_tc(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores, h1_saved,
+                                          pair_inv, k_vol, k_tgt, k_W1, k_W2, k_b2, B, N, s, (unsigned)grid, true)
+                    : launch_score_bwd(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores, k_vol, k_tgt,
+                                       k_W1, k_W2, k_b2, B, N, s, h1_saved, pair_inv, k_R, (unsigned)grid, true);
+  if (st != AHV_OK) return st;
   const int64_t n_all = kDetWSlot + (int64_t)B * kDetSegSlot + (shared_R ? N * 9 : 0);
   const unsigned blocks = (unsigned)std::min<int64_t>((n_all + 255) / 256, 8 * (int64_t)sms);
   score_bwd_det_reduce<<<blocks, 256, 0, s>>>(ws, w.seg, w.rot, grid, B, N, g_vol, g_tgt, g_W1, g_W2, g_b2,

@@ -46,9 +46,11 @@
 // kDet (ahv_score_backward_det): no float atomics - dV, dT and the weight gradients go to the workspace slots of
 // DetBwdWs (ahv_common.cuh: g_vol / g_tgt point at the segment slots, g_W1 / g_W2 / g_b2 at the weight slots) - and
 // every input voxel's contributions are summed in increasing output-voxel order: a sorting network over the row in
-// registers (oddeven_sort), an insertion sort of the exact path's lists.
+// registers, an insertion sort of the exact path's lists.  The exact path's work list, the sorts and the flushes of the
+// gradients are shared with the fp32 backward (ahv_adjoint.cuh).
 #include <cstddef>
 
+#include "ahv_adjoint.cuh"
 #include "ahv_head_fp32.cuh"
 #include "ahv_tc_ptx.cuh"
 
@@ -203,13 +205,6 @@ __device__ __forceinline__ void add4_record(uint32_t* p, float kappa, uint32_t r
                                             pack_h2(fmaf(__uint_as_float(r2), kappa, b.x), fmaf(__uint_as_float(r3), kappa, b.y)));
 }
 
-// output voxel (z*64 + y*8 + x) a thread lists for the adjoint: lane bits -> x2 x1 y2 y1 z2, warp bits and j -> the rest
-__device__ __forceinline__ int out_voxel(int t, int j) {
-  const int x = ((t & 3) << 1) | ((t >> 5) & 1), y = (((t >> 2) & 3) << 1) | ((t >> 6) & 1);
-  const int z = (((t >> 4) & 1) << 2) | (((t >> 7) & 1) << 1) | j;
-  return z * 64 + y * 8 + x;
-}
-
 // rotated volume (fp32) -> the three views of the A^T operand (fp16, pair scale `sb`)
 __device__ __forceinline__ void pack_views(BwdTcSmem& sm, float sb) {
   const int t = threadIdx.x;
@@ -354,36 +349,7 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
 #pragma unroll
     for (int c = 0; c < kC; ++c) aV[j][c] = 0.0f;
 
-  auto flush_pair = [&](int b) {  // dT and dV of pair b leave the CTA
-    if constexpr (kDet) {   // the whole segment, zeros included, into slot blockIdx.x + b
-      const size_t slot = (size_t)(blockIdx.x + b) * kDetSegSlot;
-#pragma unroll
-      for (int oo = 0; oo < 8; ++oo) {
-        g_tgt[slot + (cg2 * 8 + oo) * kP + pos] = aT[oo];
-        aT[oo] = 0.0f;
-      }
-#pragma unroll
-      for (int j = 0; j < 2; ++j)
-#pragma unroll
-        for (int c = 0; c < kC; ++c) {
-          g_vol[slot + c * kVox + t + 256 * j] = aV[j][c];
-          aV[j][c] = 0.0f;
-        }
-    } else {
-#pragma unroll
-    for (int oo = 0; oo < 8; ++oo) {
-      if (aT[oo] != 0.0f) atomicAdd(g_tgt + ((size_t)b * kO + cg2 * 8 + oo) * kP + pos, aT[oo]);
-      aT[oo] = 0.0f;
-    }
-#pragma unroll
-    for (int j = 0; j < 2; ++j)
-#pragma unroll
-      for (int c = 0; c < kC; ++c) {
-        if (aV[j][c] != 0.0f) atomicAdd(g_vol + ((size_t)b * kC + c) * kVox + t + 256 * j, aV[j][c]);
-        aV[j][c] = 0.0f;
-      }
-    }
-  };
+  auto flush = [&](int b) { flush_pair<kDet>(g_tgt, g_vol, b, aT, aV, cg2, pos, true, true); };
 
   // ---- the adjoint's work list ----
   // Output voxel vo feeds the 8 input voxels of its tap with weight w.  Turned round: every INPUT voxel gets the list
@@ -398,7 +364,7 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
   // The thread's two output voxels (one per pass) are chosen two apart in x and y and four in z across the lanes of a
   // warp, so that the taps of one warp's voxels rarely meet in the same counter.
   auto list_pass = [&](int j) {
-    const int vo = out_voxel(t, j);
+    const int vo = adjoint_out_voxel(t, j);
     const uint32_t off4 = (uint32_t)((vo >> 6) * kDxD + ((vo >> 3) & 7) * kDxH + (vo & 7) * kDxW) >> 2;   // record, in 16-byte units
     const float4 tp = sm.taps[vo];
     const int line = __float_as_int(tp.x);   // ((z0+1)*10 + (y0+1))*10 + (x0+1), corner in [-1, 7]^3
@@ -431,7 +397,7 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
   for (int64_t it = lo; it < hi; ++it) {
     const int b = (int)(it / N);
     if (b != cur_b) {
-      if (cur_b >= 0) flush_pair(cur_b);
+      if (cur_b >= 0) flush(cur_b);
       __syncthreads();
       stage_volume_interleaved(sm.vol, vol_src + (size_t)b * kC * kVox);
 #pragma unroll
@@ -493,7 +459,6 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
       uint32_t r8[8];
       tmem_ld8(tq + kColH2 + hf * 8, r8);
       tmem_ld_wait();
-#pragma unroll
       const float sc = pinv * w2s;   // undo the pair scale and both weight normalisers
 #pragma unroll
       for (int oo = 0; oo < 8; ++oo) v[oo] = fmaf(__uint_as_float(r8[oo]), sc, b2r[oo]);  // + bias
@@ -728,103 +693,28 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
 #pragma unroll
           for (int i = 0; i < kListCap; ++i) en[i] = i < nn ? __byte_perm(en[i], 0, 0x1032) : 0xffffffffu;
           sort_row(en, nmax);
-#pragma unroll
-          for (int i = 0; i < kListCap; ++i) {
-            if (i >= nmax) break;   // warp-uniform
-            if (i < nn) axpy_record(aV[j], (float)(en[i] & 0xffffu) * wq, dX + ((en[i] >> 16) << 2));
-          }
-        } else {
+        }
 #pragma unroll
         for (int i = 0; i < kListCap; ++i) {
           if (i >= nmax) break;   // warp-uniform
           if (i < nn) {
-            axpy_record(aV[j], (float)(en[i] >> 16) * wq, dX + ((en[i] & 0xffffu) << 2));
+            const uint32_t off4 = kDet ? en[i] >> 16 : en[i] & 0xffffu, w16 = kDet ? en[i] & 0xffffu : en[i] >> 16;
+            axpy_record(aV[j], (float)w16 * wq, dX + (off4 << 2));
           }
-        }
         }
       }
     } else {
       // exact path (some voxel has more than kListCap contributions): counting sort with prefix sums, 8-byte entries
       __syncthreads();
-      {
-        cnt[t] = 0;
-        cnt[t + 256] = 0;
-        __syncthreads();
-        // The thread's two output voxels are chosen two apart in x and y and four in z across the lanes of a warp, so
-        // that the taps of one warp's voxels rarely meet in the same counter (adjacent voxels share half their taps and
-        // would serialise the atomics).
-        int tgt0[2];
-        uint32_t inside[2], rank[2][4];
-        float fx[2], fy[2], fz[2];
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const int vo = out_voxel(t, j);
-          const float4 tp = sm.taps[vo];
-          const int line = __float_as_int(tp.x);   // ((z0+1)*10 + (y0+1))*10 + (x0+1), corner in [-1, 7]^3
-          const int zl = line / (kHalo * kHalo), rl = line - zl * (kHalo * kHalo), yl = rl / kHalo, xl = rl - yl * kHalo;
-          const int x0 = xl - 1, y0 = yl - 1, z0 = zl - 1;
-          fx[j] = tp.y; fy[j] = tp.z; fz[j] = tp.w;
-          tgt0[j] = z0 * 64 + y0 * 8 + x0;
-          uint32_t m = 0;
-          rank[j][0] = rank[j][1] = rank[j][2] = rank[j][3] = 0;
-#pragma unroll
-          for (int dlt = 0; dlt < 8; ++dlt) {
-            const int x = x0 + (dlt & 1), y = y0 + ((dlt >> 1) & 1), z = z0 + (dlt >> 2);
-            if ((unsigned)x < 8u && (unsigned)y < 8u && (unsigned)z < 8u) {
-              m |= 1u << dlt;   // the atomic's return value is this contribution's place in its list (<= 511: 16 bits)
-              rank[j][dlt >> 1] |= (uint32_t)atomicAdd(&cnt[tgt0[j] + (dlt >> 2) * 64 + ((dlt >> 1) & 1) * 8 + (dlt & 1)], 1) << (16 * (dlt & 1));
-            }
-          }
-          inside[j] = m;
-        }
-        __syncthreads();
-        {  // exclusive scan of the 512 counters: 2 per thread, warp scan, then the 8 warp totals
-          const int c0 = cnt[2 * t], c1 = cnt[2 * t + 1];
-          const int local = c0 + c1;
-          int incl = local;
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) {
-            const int up = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += up;
-          }
-          int* wtot = reinterpret_cast<int*>(sm.red);
-          if (lane == 31) wtot[warp] = incl;
-          __syncthreads();
-          int basep = incl - local;
-          for (int w = 0; w < warp; ++w) basep += wtot[w];
-          start[2 * t] = basep;
-          start[2 * t + 1] = basep + c0;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const int vo = out_voxel(t, j);
-          const uint32_t off = (uint32_t)((vo >> 6) * kDxD + ((vo >> 3) & 7) * kDxH + (vo & 7) * kDxW);
-#pragma unroll
-          for (int dlt = 0; dlt < 8; ++dlt)
-            if ((inside[j] >> dlt) & 1u) {
-              const int dx = dlt & 1, dy = (dlt >> 1) & 1, dz = dlt >> 2;
-              const float w = (dx ? fx[j] : 1.0f - fx[j]) * (dy ? fy[j] : 1.0f - fy[j]) * (dz ? fz[j] : 1.0f - fz[j]);
-              const int v = tgt0[j] + dz * 64 + dy * 8 + dx;
-              ent[start[v] + ((rank[j][dlt >> 1] >> (16 * (dlt & 1))) & 0xffffu)] = make_uint2(off, __float_as_uint(w));
-            }
-        }
-      }
+      build_exact_list<kDxD, kDxH, kDxW>(sm.taps, cnt, start, ent, reinterpret_cast<int*>(sm.red));
       __syncthreads();
-      if constexpr (kDet) {   // the atomics ranked each list in arrival order: sort the thread's two lists by dX offset
-#pragma unroll
-        for (int j = 0; j < 2; ++j) sort_list(ent + start[t + 256 * j], cnt[t + 256 * j]);
-      }
 #pragma unroll
       for (int j = 0; j < 2; ++j) {
         const int vi = t + 256 * j;
         const int nn = cnt[vi];
-        const uint2* e = ent + start[vi];
-#pragma unroll 2
-        for (int i = 0; i < nn; ++i) {
-          const uint2 en = e[i];
-          axpy_record(aV[j], __uint_as_float(en.y) * unscale, dX + en.x);
-        }
+        uint2* e = ent + start[vi];
+        if constexpr (kDet) sort_list(e, nn);   // the atomics ranked the list in arrival order: sort it by dX offset
+        walk_list(e, nn, [&](uint2 en) { axpy_record(aV[j], __uint_as_float(en.y) * unscale, dX + en.x); });
       }
     }
     __syncthreads();  // dX (the operand buffer), taps and the work list are re-used by the next hypothesis
@@ -842,39 +732,19 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
            ph_[5] / (hi - lo), ph_[6] / (hi - lo), ph_[7] / (hi - lo), ph_[8] / (hi - lo), ph_[9] / (hi - lo), tot / (hi - lo));
   }
 #endif
-  flush_pair(cur_b);
+  flush(cur_b);
   // weight gradients: one atomic per accumulator and CTA (kDet: one store into the CTA's weight slot)
-  const size_t wslot = kDet ? (size_t)blockIdx.x * kDetWSlot : 0;
 #pragma unroll
   for (int view = 0; view < 3; ++view)
 #pragma unroll
-    for (int oo = 0; oo < 16; ++oo) {
-      float* dst = g_W1 + wslot + (16 * hf + oo) * kK + view * 128 + 32 * qd + lane;
-      if constexpr (kDet) *dst = aW1[view][oo];
-      else atomicAdd(dst, aW1[view][oo]);
-    }
-  {
-    if (qd < 2) {
+    for (int oo = 0; oo < 16; ++oo)
+      flush_weight<kDet>(g_W1 + (16 * hf + oo) * kK + view * 128 + 32 * qd + lane, aW1[view][oo]);
+  if (qd < 2) {
 #pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        float* dst = g_W2 + wslot + (16 * qd + (lane & 15)) * kO + 16 * (lane >> 4) + 8 * hf + i;
-        if constexpr (kDet) *dst = aW2[i];
-        else atomicAdd(dst, aW2[i]);
-      }
-    }
-    // db2: sum over the 64 positions inside the CTA first (threads with equal cg2 = t & 3)
-    __syncthreads();
-    float* red = sm.dh2;  // [4 cg2][8 oo][64 pos]
-#pragma unroll
-    for (int oo = 0; oo < 8; ++oo) red[(cg2 * 8 + oo) * kP + pos] = ab2[oo];
-    __syncthreads();
-    if (t < kO) {
-      float s = 0.0f;
-      for (int p = 0; p < kP; ++p) s += red[t * kP + p];
-      if constexpr (kDet) g_b2[wslot + t] = s;
-      else atomicAdd(g_b2 + t, s);
-    }
+    for (int i = 0; i < 8; ++i)
+      flush_weight<kDet>(g_W2 + (16 * qd + (lane & 15)) * kO + 16 * (lane >> 4) + 8 * hf + i, aW2[i]);
   }
+  flush_b2<kDet>(sm.dh2, ab2, cg2, pos, g_b2, true);   // sm.dh2: [4 cg2][8 oo][64 pos]
   tc_fence_before();
   __syncthreads();
   if (warp == 0) {
@@ -888,35 +758,21 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
 int launch_score_bwd_tc(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
                         const float* W1, const float* W2, const float* b2, const float* base,
                         const float* grad_scores, const void* h1_saved, const float* pair_inv, float* g_vol,
-                        float* g_tgt, float* g_W1, float* g_W2, float* g_b2, int B, int64_t N, cudaStream_t s) {
+                        float* g_tgt, float* g_W1, float* g_W2, float* g_b2, int B, int64_t N, cudaStream_t s,
+                        unsigned grid, bool det) {
   const int64_t total = (int64_t)B * N;
   if (total == 0) return AHV_OK;
   if (!h1_saved || !pair_inv) return AHV_EINVAL;
-  int dev = 0, sms = 0;
-  AHV_CUDA_OK(cudaGetDevice(&dev));
-  AHV_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  const unsigned grid = (unsigned)(total < sms ? total : sms);
+  if (grid == 0) {
+    const int sms = sm_count();
+    if (sms <= 0) return AHV_ECUDA;
+    grid = (unsigned)(total < sms ? total : sms);
+  }
+  const auto kernel = det ? score_bwd_tc_kernel<true> : score_bwd_tc_kernel<false>;
   const size_t smem = sizeof(BwdTcSmem);
-  AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  score_bwd_tc_kernel<false><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
-                                                   static_cast<const __half*>(h1_saved), pair_inv, g_vol, g_tgt,
-                                                   g_W1, g_W2, g_b2, B, N);
-  AHV_CUDA_OK(cudaGetLastError());
-  return AHV_OK;
-}
-
-// the kDet instance on `grid` CTAs (launch_score_bwd_det picks it and reduces the slots)
-int launch_score_bwd_tc_det(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
-                            const float* W1, const float* W2, const float* b2, const float* base,
-                            const float* grad_scores, const void* h1_saved, const float* pair_inv, float* ws_w,
-                            float* ws_seg, int B, int64_t N, unsigned grid, cudaStream_t s) {
-  if (!h1_saved || !pair_inv) return AHV_EINVAL;
-  const size_t smem = sizeof(BwdTcSmem);
-  AHV_CUDA_OK(cudaFuncSetAttribute(score_bwd_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  score_bwd_tc_kernel<true><<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
-                                                         static_cast<const __half*>(h1_saved), pair_inv, ws_seg,
-                                                         ws_seg + kC * kVox, ws_w, ws_w + kO * kK, ws_w + kO * kK + kO * kO,
-                                                         B, N);
+  AHV_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
+                                      static_cast<const __half*>(h1_saved), pair_inv, g_vol, g_tgt, g_W1, g_W2, g_b2, B, N);
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }

@@ -263,12 +263,6 @@ int launch_rotate_volume_grad_R(const float* vol, int per_rot, const float* R, c
 }
 
 // ---- launchers --------------------------------------------------------------
-static int sm_count() {
-  int dev = 0, sms = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
-  return sms;
-}
 
 int launch_score_fp32(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R,
                       int r_per_pair, const float* W1, const float* W2, const float* b2,

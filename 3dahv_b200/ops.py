@@ -244,18 +244,14 @@ def score_backward(vol_src: torch.Tensor, tgt_feat: torch.Tensor, R: torch.Tenso
               W2.data_ptr(), b2.data_ptr(), base_coords(dev).data_ptr(), gs.data_ptr(), ptr(h1), ptr(pi),
               *(ptr(t) for t in outs), B, N, mode, workspace.data_ptr(), ws_bytes)
         return outs if want_grad_R else outs[:5]
-    if want_grad_R:
-        g_R = z(*R.shape)
-        _score_backward_ex(vs, tg, R, W1, W2, b2, gs, h1, pi, (g_vol, g_tgt, g_w1, g_w2, g_b2, g_R), B, N, per_pair)
-        return g_vol, g_tgt, g_w1, g_w2, g_b2, g_R
-    head = (vs.data_ptr(), tg.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
-            base_coords(dev).data_ptr(), gs.data_ptr())
-    tail = (g_vol.data_ptr(), g_tgt.data_ptr(), g_w1.data_ptr(), g_w2.data_ptr(), g_b2.data_ptr(), B, N)
-    if h1 is not None:
-        _call("ahv_score_backward_saved", dev, *head, h1.data_ptr(), pi.data_ptr(), *tail, int(math))
-    else:
-        _call("ahv_score_backward", dev, *head, *tail)
-    return g_vol, g_tgt, g_w1, g_w2, g_b2
+    if h1 is not None and not want_grad_R and math != MATH_FP32:   # the tcgen05 kernel (the entry checks `math`)
+        _call("ahv_score_backward_saved", dev, vs.data_ptr(), tg.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(),
+              W2.data_ptr(), b2.data_ptr(), base_coords(dev).data_ptr(), gs.data_ptr(), h1.data_ptr(), pi.data_ptr(),
+              g_vol.data_ptr(), g_tgt.data_ptr(), g_w1.data_ptr(), g_w2.data_ptr(), g_b2.data_ptr(), B, N, int(math))
+        return g_vol, g_tgt, g_w1, g_w2, g_b2
+    g_R = z(*R.shape) if want_grad_R else None
+    _score_backward_ex(vs, tg, R, W1, W2, b2, gs, h1, pi, (g_vol, g_tgt, g_w1, g_w2, g_b2, g_R), B, N, per_pair)
+    return (g_vol, g_tgt, g_w1, g_w2, g_b2, g_R) if want_grad_R else (g_vol, g_tgt, g_w1, g_w2, g_b2)
 
 
 def score_backward_det_workspace_bytes(B: int, N: int, per_pair: bool, want_grad_R: bool) -> int:

@@ -318,8 +318,9 @@ def test_paths_without_a_deterministic_form_alert_under_the_flag(ahv, golden, mo
     chunked()
 
 
-def test_the_flag_picks_the_entry(ahv, golden, monkeypatch):
-    """Without the flag the training path calls the atomic entries exactly as before; with it, the deterministic one."""
+def test_the_flag_picks_the_atomic_or_deterministic_entry(ahv, golden, monkeypatch):
+    """Without the flag the training path calls the atomic entries: ahv_score_backward_saved for saved activations on
+    tcgen05, ahv_score_backward_ex for every other form; with it, the deterministic one."""
     monkeypatch.setenv("CUBLAS_WORKSPACE_CONFIG", ":4096:8")   # the head's matmuls under the flag
     args = _inputs(ahv, golden, 2, 30, True, seed=31)
     vs, tgt, R, W1, W2, b2, gs = args
@@ -336,7 +337,7 @@ def test_the_flag_picks_the_entry(ahv, golden, monkeypatch):
         (s * gs).sum().backward()
         return [c for c in called if c.startswith("ahv_score_backward")]
 
-    expect_atomic = {(False, False): "ahv_score_backward", (True, False): "ahv_score_backward_saved",
+    expect_atomic = {(False, False): "ahv_score_backward_ex", (True, False): "ahv_score_backward_saved",
                      (False, True): "ahv_score_backward_ex", (True, True): "ahv_score_backward_ex"}
     for (save, want_R), name in expect_atomic.items():
         assert step(save, want_R) == [name], (save, want_R)
