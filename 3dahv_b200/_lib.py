@@ -56,6 +56,9 @@ SIGNATURES = {
     "ahv_topk_distinct": (_i, [_vp, _vp, _i, _i, _i64, _i, ctypes.c_float, _vp, _vp, _vp, _vp]),
     "ahv_posterior_mass_workspace_bytes": (_sz, [_i, _i64, _i]),
     "ahv_posterior_mass": (_i, [_vp, _vp, _i, _vp, _i, _i64, _i, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp, _sz, _vp]),
+    "ahv_posterior_moments_workspace_bytes": (_sz, [_i, _i64, _i]),
+    "ahv_posterior_moments": (_i, [_vp, _vp, _i, _vp, _i, _i64, _i, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp, _vp, _vp,
+                                   _vp, _sz, _vp]),
     "ahv_topk": (_i, [_vp, _i, _i64, _i, _i64, _vp, _vp, _vp, _sz, _vp]),
     "ahv_topk_merge": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "ahv_gather_rotations": (_i, [_vp, _i, _vp, _i64, _i, _i64, _i, _vp, _vp]),

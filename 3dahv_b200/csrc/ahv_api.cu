@@ -532,7 +532,7 @@ bool posterior_sizes_ok(int B, int64_t N, int k) { return B >= 0 && N >= 1 && n_
 }  // namespace
 
 AHV_API size_t ahv_posterior_mass_workspace_bytes(int B, int64_t N, int k) {
-  return posterior_sizes_ok(B, N, k) ? posterior_workspace_bytes(B, N, k) : 0;
+  return posterior_sizes_ok(B, N, k) ? posterior_workspace_bytes(B, N, k, false) : 0;
 }
 
 AHV_API int ahv_posterior_mass(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N,
@@ -543,11 +543,31 @@ AHV_API int ahv_posterior_mass(const float* scores, const float* R, int r_per_pa
   if (B > 0 && !all_set(scores, R, log_z, workspace)) return AHV_EINVAL;
   if (k > 0 ? (B > 0 && !all_set(centers, mass)) : (centers || mass)) return AHV_EINVAL;  // k == 0: log_z alone
   if (!all_aligned16(R, centers, workspace)) return AHV_EINVAL;
-  if (B > 0 && workspace_bytes < posterior_workspace_bytes(B, N, k)) return AHV_EWORKSPACE;
+  if (B > 0 && workspace_bytes < posterior_workspace_bytes(B, N, k, false)) return AHV_EWORKSPACE;
   int st = check_device();
   if (st != AHV_OK) return st;
-  return launch_posterior_mass(scores, R, r_per_pair != 0, centers, B, N, k, radius_deg, temperature, log_z, mass, workspace,
-                               (cudaStream_t)stream);
+  return launch_posterior(scores, R, r_per_pair != 0, centers, B, N, k, radius_deg, temperature, log_z, mass, nullptr,
+                          nullptr, nullptr, workspace, (cudaStream_t)stream);
+}
+
+// ---- first moment of the posterior over each slot: mean rotation and spread (extension) ------------------
+AHV_API size_t ahv_posterior_moments_workspace_bytes(int B, int64_t N, int k) {
+  return posterior_sizes_ok(B, N, k) && k_ok(k) ? posterior_workspace_bytes(B, N, k, true) : 0;
+}
+
+AHV_API int ahv_posterior_moments(const float* scores, const float* R, int r_per_pair, const float* centers, int B,
+                                  int64_t N, int k, float radius_deg, float temperature, float* log_z, float* mass,
+                                  float* mean_R, float* mean_cos, float* moment, void* workspace,
+                                  size_t workspace_bytes, void* stream) {
+  if (!posterior_sizes_ok(B, N, k) || !k_ok(k) || !min_sep_ok(radius_deg)) return AHV_EINVAL;
+  if (!std::isfinite(temperature) || !(temperature > 0.0f)) return AHV_EINVAL;
+  if (B > 0 && !all_set(scores, R, centers, log_z, mass, mean_R, mean_cos, moment, workspace)) return AHV_EINVAL;
+  if (!all_aligned16(R, centers, workspace)) return AHV_EINVAL;
+  if (B > 0 && workspace_bytes < posterior_workspace_bytes(B, N, k, true)) return AHV_EWORKSPACE;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  return launch_posterior(scores, R, r_per_pair != 0, centers, B, N, k, radius_deg, temperature, log_z, mass, mean_R,
+                          mean_cos, moment, workspace, (cudaStream_t)stream);
 }
 
 // ---- hypothesis set sharded over the GPUs of one node: winners exchanged through peer memory -------------

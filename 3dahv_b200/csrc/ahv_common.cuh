@@ -257,8 +257,10 @@ struct ScreenLists {  // carved from the verification workspace's top-k partials
 int launch_screen_select(const float* s16, const unsigned long long* keys, int B, int64_t N, const float* R, int r_per_pair,
                          const ScreenLists& L, float* R_list, cudaStream_t s);
 int launch_screen_guard(const float* s32, const ScreenLists& L, int B, unsigned long long* keys, cudaStream_t s);
-size_t posterior_workspace_bytes(int B, int64_t N, int k);
-int launch_posterior_mass(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N, int k,
-                          float radius_deg, float temperature, float* log_z, float* mass, void* ws, cudaStream_t s);
+size_t posterior_workspace_bytes(int B, int64_t N, int k, bool moments);
+// ahv_posterior_mass (moment == nullptr) and ahv_posterior_moments (mean_R, mean_cos and moment set)
+int launch_posterior(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N, int k,
+                     float radius_deg, float temperature, float* log_z, float* mass, float* mean_R, float* mean_cos,
+                     float* moment, void* ws, cudaStream_t s);
 
 }  // namespace ahv

@@ -196,6 +196,14 @@ int launch_topk_distinct(const float* scores, const float* R, int r_per_pair, in
 // warps in order; a chunk holding a NaN or +inf score records m_c = NaN.  Pass 2, one CTA per pair: m = max m_c
 // (exact), then every sum rescaled by exp((m_c - m)/T) and added over the chunks in a fixed tree, each cast to fp32
 // once.  Workspace: [the chunk sums, B*chunks*(k+1) doubles | the chunk maxima, B*chunks floats].
+//
+// With kMoments (ahv_posterior_moments; DESIGN.md §4.7.1) the same two launches also form each slot's first moment
+// M_j = sum_{n -> j} e_n R_n / W_j (W_j = the mass's own unnormalised sum) and project it onto SO(3).  Pass 1: every
+// thread remembers the slot of each of its kPer hypotheses (a byte); per slot that some lane of the warp holds, each
+// lane sums e_n R_n over its own hits in index order (re-reading R_n through L1/L2), a butterfly adds the lanes, and
+// the warps are added in order into the chunk's record of k*9 doubles.  Pass 2: one warp per slot rescales the records
+// with the mass's factors exp((m_c - m)/T) and adds them over the chunks (lane-strided, then the butterfly), divides by
+// W_j, and slot j's thread projects M_j (q-method, project_so3).  Workspace: the mass's, then B*chunks*k*9 doubles.
 namespace posterior {
 constexpr int kThreads = 128;
 constexpr int kWarps = kThreads / 32;
@@ -209,10 +217,55 @@ __device__ __forceinline__ double warp_sum_d(double v) {
   return v;
 }
 
+// Slot j's record of the chunk, out[j*9 + q] = sum_{n -> j} e_n R_n[q]: per lane over its own hits in index order (s_n
+// and R_n re-read through L1/L2, e_n recomputed as the mass formed it), then the warp butterfly, then the warps in
+// order.  A slot no lane of the warp holds adds zeros.
+__device__ __forceinline__ void chunk_moments(const uint8_t (&slot)[kPer], unsigned held, float mx, double T,
+                                              const float* __restrict__ row, const float* __restrict__ Rp, int64_t first,
+                                              int k, double* __restrict__ out) {
+  __shared__ double s_mom[kMaxK][kWarps][9];
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  const unsigned warp_held = __reduce_or_sync(0xffffffffu, held);
+  for (int j = 0; j < k; ++j) {
+    double a[9];
+#pragma unroll
+    for (int q = 0; q < 9; ++q) a[q] = 0.0;
+    if ((warp_held >> j) & 1u) {
+      unsigned hits = 0u;  // bit i: the thread's i-th hypothesis is in slot j
+#pragma unroll
+      for (int i = 0; i < kPer; ++i) hits |= (unsigned)(slot[i] == j) << i;
+      while (hits) {
+        const int i = __ffs(hits) - 1;
+        hits &= hits - 1;
+        const int64_t n = first + i * kThreads + t;
+        const double e = exp(((double)__ldg(row + n) - (double)mx) / T);
+        const float* Rn = Rp + (size_t)n * 9;
+#pragma unroll
+        for (int q = 0; q < 9; ++q) a[q] += e * (double)__ldg(Rn + q);
+      }
+#pragma unroll
+      for (int q = 0; q < 9; ++q) a[q] = warp_sum_d(a[q]);
+    }
+    if (lane == 0) {
+#pragma unroll
+      for (int q = 0; q < 9; ++q) s_mom[j][warp][q] = a[q];
+    }
+  }
+  __syncthreads();
+  for (int v = t; v < k * 9; v += kThreads) {
+    const int j = v / 9, q = v % 9;
+    double x = s_mom[j][0][q];
+#pragma unroll
+    for (int w = 1; w < kWarps; ++w) x += s_mom[j][w][q];
+    out[v] = x;
+  }
+}
+
+template <bool kMoments>
 __global__ void __launch_bounds__(kThreads)
 posterior_chunk_kernel(const float* __restrict__ scores, const float* __restrict__ R, int r_per_pair,
                        const float* __restrict__ centers, int B, int64_t N, int k, float c, double T, int chunks,
-                       double* __restrict__ ws_sum, float* __restrict__ ws_max) {
+                       double* __restrict__ ws_sum, float* __restrict__ ws_max, double* __restrict__ ws_mom) {
   __shared__ double s_acc[kMaxK * kThreads];  // slot j of thread t at [j][t]: each thread adds into its own column
   __shared__ double s_red[kMaxK + 1][kWarps];
   __shared__ float s_cen[kMaxK][9];
@@ -249,6 +302,12 @@ posterior_chunk_kernel(const float* __restrict__ scores, const float* __restrict
       bad |= s_wbad[w] != 0;
     }
     double tot = 0.0;
+    [[maybe_unused]] uint8_t slot[kPer];  // kMoments: the slot of each of the thread's hypotheses (0xFF: none)
+    [[maybe_unused]] unsigned held = 0u;  // kMoments: bit j set when the thread holds a hypothesis of slot j
+    if constexpr (kMoments) {
+#pragma unroll
+      for (int i = 0; i < kPer; ++i) slot[i] = 0xFF;
+    }
     if (!bad) {
 #pragma unroll
       for (int i = 0; i < kPer; ++i) {
@@ -264,6 +323,10 @@ posterior_chunk_kernel(const float* __restrict__ scores, const float* __restrict
           for (int j = 0; j < k; ++j) {
             if (distinct::trace_rn(a, s_cen[j]) >= c) {  // a NaN trace (empty slot) never passes
               s_acc[j * kThreads + t] += e;
+              if constexpr (kMoments) {
+                slot[i] = (uint8_t)j;
+                held |= 1u << j;
+              }
               break;
             }
           }
@@ -283,14 +346,145 @@ posterior_chunk_kernel(const float* __restrict__ scores, const float* __restrict
       ws_sum[rec * (k + 1) + t] = x;
     }
     if (t == 0) ws_max[rec] = bad ? NAN : mx;
+    if constexpr (kMoments) chunk_moments(slot, held, mx, T, row, Rp, first, k, ws_mom + rec * k * 9);
     __syncthreads();  // the next pair reuses the shared arrays
   }
 }
 
+constexpr int kFinalW = kFinalThreads / 32;
+constexpr int kJacobiSweeps = 8;  // at most; 4-5 cyclic sweeps bring a 4x4 to diagonal in double
+
+// R = argmax_{R in SO(3)} tr(R^T M) by the q-method (Horn 1987, Davenport): for R = R(w, x, y, z), tr(R^T M) = q^T K q
+// with K below, so R's unit quaternion is K's eigenvector of the largest eigenvalue (any of them on a tie) and
+// R(q) is a proper rotation by construction.  K is diagonalised by cyclic Jacobi in double, at most kJacobiSweeps
+// sweeps, stopping once the off-diagonal squares sum to at most 1e-32 of the diagonal's: the result depends on M
+// alone.  Returns tr(R^T M).  Row-major 3x3.
+__host__ __device__ inline double project_so3(const double (&M)[9], double (&Rout)[9]) {
+  double a[4][4] = {{M[0] + M[4] + M[8], M[7] - M[5], M[2] - M[6], M[3] - M[1]},
+                    {M[7] - M[5], M[0] - M[4] - M[8], M[1] + M[3], M[2] + M[6]},
+                    {M[2] - M[6], M[1] + M[3], -M[0] + M[4] - M[8], M[5] + M[7]},
+                    {M[3] - M[1], M[2] + M[6], M[5] + M[7], -M[0] - M[4] + M[8]}};
+  double v[4][4] = {{1, 0, 0, 0}, {0, 1, 0, 0}, {0, 0, 1, 0}, {0, 0, 0, 1}};
+#pragma unroll 1
+  for (int sweep = 0; sweep < kJacobiSweeps; ++sweep) {
+    double off = 0.0, diag = 0.0;
+#pragma unroll
+    for (int p = 0; p < 4; ++p) {
+      diag += a[p][p] * a[p][p];
+#pragma unroll
+      for (int q = p + 1; q < 4; ++q) off += a[p][q] * a[p][q];
+    }
+    if (off <= 1e-32 * diag) break;
+#pragma unroll
+    for (int p = 0; p < 3; ++p) {
+#pragma unroll
+      for (int q = p + 1; q < 4; ++q) {
+        if (a[p][q] == 0.0) continue;
+        // Golub & Van Loan, sym.schur2: J = [c s; -s c] on (p, q) zeroes a[p][q] of J^T A J
+        const double tau = (a[q][q] - a[p][p]) / (2.0 * a[p][q]);
+        const double t = (tau >= 0.0 ? 1.0 : -1.0) / (fabs(tau) + sqrt(1.0 + tau * tau));
+        const double cs = 1.0 / sqrt(1.0 + t * t), sn = t * cs;
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+          const double ap = a[r][p], aq = a[r][q];
+          a[r][p] = cs * ap - sn * aq;
+          a[r][q] = sn * ap + cs * aq;
+        }
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+          const double ap = a[p][r], aq = a[q][r];
+          a[p][r] = cs * ap - sn * aq;
+          a[q][r] = sn * ap + cs * aq;
+        }
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+          const double vp = v[r][p], vq = v[r][q];
+          v[r][p] = cs * vp - sn * vq;
+          v[r][q] = sn * vp + cs * vq;
+        }
+      }
+    }
+  }
+  double best = a[0][0], w = v[0][0], x = v[1][0], y = v[2][0], z = v[3][0];
+#pragma unroll
+  for (int e = 1; e < 4; ++e) {
+    if (a[e][e] > best) {
+      best = a[e][e];
+      w = v[0][e], x = v[1][e], y = v[2][e], z = v[3][e];
+    }
+  }
+  const double inv = 1.0 / sqrt(w * w + x * x + y * y + z * z);
+  w *= inv, x *= inv, y *= inv, z *= inv;
+  Rout[0] = w * w + x * x - y * y - z * z, Rout[1] = 2.0 * (x * y - w * z), Rout[2] = 2.0 * (x * z + w * y);
+  Rout[3] = 2.0 * (x * y + w * z), Rout[4] = w * w - x * x + y * y - z * z, Rout[5] = 2.0 * (y * z - w * x);
+  Rout[6] = 2.0 * (x * z - w * y), Rout[7] = 2.0 * (y * z + w * x), Rout[8] = w * w - x * x - y * y + z * z;
+  double tr = 0.0;
+#pragma unroll
+  for (int e = 0; e < 9; ++e) tr += Rout[e] * M[e];
+  return tr;
+}
+
+// Pass 2 of the moments, after the mass.  Warp w takes slots w, w + 8, ...: each lane adds the slot's records of chunks
+// lane, lane + 32, ... in index order, rescaled by the mass's factors exp((m_c - m)/T), then the butterfly; the sums are
+// divided by W_j (the mass's own sum of slot j, re-added from s_red in the mass's order).  Then slot j's thread projects
+// M_j.  A pair with a NaN or +inf score, and a slot with W_j = 0, get NaN.
+__device__ __forceinline__ void final_moments(const double* __restrict__ rec, const float* __restrict__ mc, int chunks, int k,
+                                              double T, float m, bool live, bool bad, const double (*s_red)[kFinalW],
+                                              float* __restrict__ mean_R, float* __restrict__ mean_cos,
+                                              float* __restrict__ moment) {
+  __shared__ double s_M[kMaxK][9];
+  const int b = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  for (int j = warp; j < k; j += kFinalW) {
+    double a[9];
+#pragma unroll
+    for (int q = 0; q < 9; ++q) a[q] = 0.0;
+    if (live) {
+      for (int i = lane; i < chunks; i += 32) {
+        const float mi = mc[i];
+        if (mi == -INFINITY) continue;  // the chunk holds nothing (its records are 0)
+        const double f = exp(((double)mi - (double)m) / T);
+        const double* r = rec + ((size_t)i * k + j) * 9;
+#pragma unroll
+        for (int q = 0; q < 9; ++q) a[q] += r[q] * f;
+      }
+    }
+#pragma unroll
+    for (int q = 0; q < 9; ++q) a[q] = warp_sum_d(a[q]);
+    if (lane == 0) {
+      double W = s_red[j + 1][0];
+#pragma unroll
+      for (int w = 1; w < kFinalW; ++w) W += s_red[j + 1][w];
+#pragma unroll
+      for (int q = 0; q < 9; ++q) {
+        const double M = !bad && W > 0.0 ? a[q] / W : (double)NAN;
+        s_M[j][q] = M;
+        moment[((size_t)b * k + j) * 9 + q] = (float)M;
+      }
+    }
+  }
+  __syncthreads();
+  if (t < k) {
+    double M[9], Rb[9];
+    bool nan = false;
+#pragma unroll
+    for (int e = 0; e < 9; ++e) {
+      M[e] = s_M[t][e];
+      nan |= isnan(M[e]);
+    }
+    const double tr = project_so3(M, Rb);
+    float* out = mean_R + ((size_t)b * k + t) * 9;
+#pragma unroll
+    for (int e = 0; e < 9; ++e) out[e] = nan ? NAN : (float)Rb[e];
+    mean_cos[(size_t)b * k + t] = nan ? NAN : (float)fmin(fmax((tr - 1.0) * 0.5, -1.0), 1.0);
+  }
+}
+
+template <bool kMoments>
 __global__ void __launch_bounds__(kFinalThreads)
 posterior_final_kernel(const double* __restrict__ ws_sum, const float* __restrict__ ws_max, int chunks, int k, double T,
-                       float* __restrict__ log_z, float* __restrict__ mass) {
-  constexpr int kW = kFinalThreads / 32;
+                       float* __restrict__ log_z, float* __restrict__ mass, const double* __restrict__ ws_mom,
+                       float* __restrict__ mean_R, float* __restrict__ mean_cos, float* __restrict__ moment) {
+  constexpr int kW = kFinalW;
   __shared__ float s_wmax[kW];
   __shared__ int s_wbad[kW];
   __shared__ double s_red[kMaxK + 1][kW];
@@ -341,33 +535,51 @@ posterior_final_kernel(const double* __restrict__ ws_sum, const float* __restric
     if (t == 0) log_z[b] = bad ? NAN : (float)((double)m / T + log(S));
     else mass[(size_t)b * k + t - 1] = bad ? NAN : (float)(S / Z);
   }
+  if constexpr (kMoments)
+    final_moments(ws_mom + (size_t)b * chunks * k * 9, mc, chunks, k, T, m, live, bad, s_red, mean_R, mean_cos, moment);
 }
 
 struct Ws {
   int chunks;
-  size_t max, total;  // byte offsets: the sums at 0, the maxima at `max`
-  Ws(int B, int64_t N, int k)
+  size_t max, mom, total;  // byte offsets: the sums at 0, the maxima at `max`, the moment records (kMoments) at `mom`
+  Ws(int B, int64_t N, int k, bool moments)
       : chunks((int)((N + kChunk - 1) / kChunk)),
         max(((size_t)B * chunks * (k + 1) * sizeof(double) + 255) / 256 * 256),
-        total(max + ((size_t)B * chunks * sizeof(float) + 255) / 256 * 256) {}
+        mom(max + ((size_t)B * chunks * sizeof(float) + 255) / 256 * 256),
+        total(mom + (moments ? ((size_t)B * chunks * k * 9 * sizeof(double) + 255) / 256 * 256 : 0)) {}
 };
 }  // namespace posterior
 
-size_t posterior_workspace_bytes(int B, int64_t N, int k) { return posterior::Ws(B, N, k).total; }
+size_t posterior_workspace_bytes(int B, int64_t N, int k, bool moments) { return posterior::Ws(B, N, k, moments).total; }
 
-int launch_posterior_mass(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N, int k,
-                          float radius_deg, float temperature, float* log_z, float* mass, void* ws, cudaStream_t s) {
+int launch_posterior(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N, int k,
+                     float radius_deg, float temperature, float* log_z, float* mass, float* mean_R, float* mean_cos,
+                     float* moment, void* ws, cudaStream_t s) {
   using namespace posterior;
   if (B == 0) return AHV_OK;
-  const Ws w(B, N, k);
+  const bool moments = moment != nullptr;
+  const Ws w(B, N, k, moments);
   double* ws_sum = static_cast<double*>(ws);
   float* ws_max = reinterpret_cast<float*>(static_cast<unsigned char*>(ws) + w.max);
-  const unsigned pairs = (unsigned)(B < 65535 ? B : 65535);
-  posterior_chunk_kernel<<<dim3((unsigned)w.chunks, pairs), kThreads, 0, s>>>(
-      scores, R, r_per_pair, centers, B, N, k, distinct::trace_threshold(radius_deg), (double)temperature, w.chunks, ws_sum,
-      ws_max);
+  double* ws_mom = moments ? reinterpret_cast<double*>(static_cast<unsigned char*>(ws) + w.mom) : nullptr;
+  const dim3 grid1((unsigned)w.chunks, (unsigned)(B < 65535 ? B : 65535));
+  const float c = distinct::trace_threshold(radius_deg);
+  const double T = (double)temperature;
+  if (moments) {
+    posterior_chunk_kernel<true><<<grid1, kThreads, 0, s>>>(scores, R, r_per_pair, centers, B, N, k, c, T, w.chunks, ws_sum,
+                                                            ws_max, ws_mom);
+  } else {
+    posterior_chunk_kernel<false><<<grid1, kThreads, 0, s>>>(scores, R, r_per_pair, centers, B, N, k, c, T, w.chunks,
+                                                             ws_sum, ws_max, nullptr);
+  }
   AHV_CUDA_OK(cudaGetLastError());
-  posterior_final_kernel<<<(unsigned)B, kFinalThreads, 0, s>>>(ws_sum, ws_max, w.chunks, k, (double)temperature, log_z, mass);
+  if (moments) {
+    posterior_final_kernel<true><<<(unsigned)B, kFinalThreads, 0, s>>>(ws_sum, ws_max, w.chunks, k, T, log_z, mass, ws_mom,
+                                                                       mean_R, mean_cos, moment);
+  } else {
+    posterior_final_kernel<false><<<(unsigned)B, kFinalThreads, 0, s>>>(ws_sum, ws_max, w.chunks, k, T, log_z, mass,
+                                                                        nullptr, nullptr, nullptr, nullptr);
+  }
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }

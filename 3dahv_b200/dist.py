@@ -279,11 +279,11 @@ class ShardedVerifier:
 
     @torch.no_grad()
     def posterior(self, vol_src, vol_tgt, R, k: int = 1, min_sep_deg: float = 0.0, radius_deg: float | None = None,
-                  temperature: float = 0.1, R_query=None):
+                  temperature: float = 0.1, R_query=None, moments: bool = False):
         """`HypothesisVerifier.posterior` over a sharded set: every rank passes the WHOLE set and gets the one-GPU
         result bit for bit.  The slices' scores are assembled into the whole [B,N] on every rank (`scores`, as for the
-        distinct selection), and the selection and `ops.posterior_mass` run replicated on every rank; R_query's few
-        rotations are scored on every rank."""
+        distinct selection), and the selection and `ops.posterior_mass` (`ops.posterior_moments` with moments) run
+        replicated on every rank; R_query's few rotations are scored on every rank."""
         from .verify import _posterior, _posterior_radius, _src_volume
 
         radius_deg = _posterior_radius(min_sep_deg, radius_deg)
@@ -294,7 +294,7 @@ class ShardedVerifier:
             v = self.verifier
             W1, W2, b2 = v._weights_on(vol_src.device)
             s_query = ops.score(_src_volume(vol_src), v.target_features(vol_tgt), R_query, W1, W2, b2, k=0, math=v.math)[0]
-        return _posterior(scores, R, min(k, N), min_sep_deg, radius_deg, temperature, s_query)
+        return _posterior(scores, R, min(k, N), min_sep_deg, radius_deg, temperature, s_query, moments)
 
     @torch.no_grad()
     def scores(self, vol_src, vol_tgt, R):

@@ -625,14 +625,8 @@ def posterior_mass_workspace_bytes(B: int, N: int, k: int) -> int:
     return int(_lib.lib().ahv_posterior_mass_workspace_bytes(B, N, k))
 
 
-def posterior_mass(scores: torch.Tensor, R: torch.Tensor, centers: torch.Tensor | None, radius_deg: float,
-                   temperature: float = 0.1, workspace: torch.Tensor | None = None):
-    """ahv_posterior_mass: the softmax p_b(n) = exp(scores[b,n]/T) / Z_b over the hypothesis set, summarised per pair.
-    Returns (log_z [B] = log Z_b, mass [B,k]): mass[b,j] is the probability of the hypotheses whose lowest slot j with
-    trace(R_n c_j^T) >= fp32(1 + 2 cos(radius_deg)) is j - `topk_distinct`'s trace test, so with centers = its R_best
-    and radius_deg = its min_sep_deg, slot j holds its winner and the hypotheses that winner suppressed.  scores [B,N];
-    R [N,3,3] or [B,N,3,3]; centers [B,k,3,3] (NaN = empty slot, mass 0) or None (k = 0: mass is [B,0]).  A pair with a
-    NaN or +inf score gets NaN outputs.  Deterministic, bit-identical whatever the batch around a pair."""
+def _posterior_args(scores, R, centers):
+    """The checks `posterior_mass` and `posterior_moments` share: (scores, R, per_pair, centers or None)."""
     s, R = _dev(scores, "scores"), _dev(R, "R")
     B, N = s.shape
     per_pair = R.dim() == 4
@@ -643,6 +637,19 @@ def posterior_mass(scores: torch.Tensor, R: torch.Tensor, centers: torch.Tensor 
         c = _dev(centers, "centers")
         if c.dim() != 4 or c.shape[0] != B or tuple(c.shape[2:]) != (3, 3):
             raise ValueError("centers must be [B,k,3,3]")
+    return s, R, per_pair, c
+
+
+def posterior_mass(scores: torch.Tensor, R: torch.Tensor, centers: torch.Tensor | None, radius_deg: float,
+                   temperature: float = 0.1, workspace: torch.Tensor | None = None):
+    """ahv_posterior_mass: the softmax p_b(n) = exp(scores[b,n]/T) / Z_b over the hypothesis set, summarised per pair.
+    Returns (log_z [B] = log Z_b, mass [B,k]): mass[b,j] is the probability of the hypotheses whose lowest slot j with
+    trace(R_n c_j^T) >= fp32(1 + 2 cos(radius_deg)) is j - `topk_distinct`'s trace test, so with centers = its R_best
+    and radius_deg = its min_sep_deg, slot j holds its winner and the hypotheses that winner suppressed.  scores [B,N];
+    R [N,3,3] or [B,N,3,3]; centers [B,k,3,3] (NaN = empty slot, mass 0) or None (k = 0: mass is [B,0]).  A pair with a
+    NaN or +inf score gets NaN outputs.  Deterministic, bit-identical whatever the batch around a pair."""
+    s, R, per_pair, c = _posterior_args(scores, R, centers)
+    B, N = s.shape
     k = 0 if c is None else c.shape[1]
     log_z = torch.empty(B, device=s.device, dtype=torch.float32)
     mass = torch.empty(B, k, device=s.device, dtype=torch.float32)
@@ -651,6 +658,35 @@ def posterior_mass(scores: torch.Tensor, R: torch.Tensor, centers: torch.Tensor 
           float(radius_deg), float(temperature), log_z.data_ptr(), mass.data_ptr() if k else None, workspace.data_ptr(),
           ws_bytes)
     return log_z, mass
+
+
+def posterior_moments_workspace_bytes(B: int, N: int, k: int) -> int:
+    """Bytes of scratch `posterior_moments` needs (0 for invalid sizes)."""
+    return int(_lib.lib().ahv_posterior_moments_workspace_bytes(B, N, k))
+
+
+def posterior_moments(scores: torch.Tensor, R: torch.Tensor, centers: torch.Tensor, radius_deg: float,
+                      temperature: float = 0.1, workspace: torch.Tensor | None = None):
+    """ahv_posterior_moments: `posterior_mass` (the same slots, and log_z and mass bit for bit) and the first moment of
+    p_b over each slot.  Returns (log_z [B], mass [B,k], mean_R [B,k,3,3], mean_cos [B,k], moment [B,k,3,3]):
+    moment[b,j] = M_j, the p-weighted mean of the hypothesis matrices in slot j; mean_R[b,j] = argmax over SO(3) of
+    tr(R^T M_j), a proper rotation; mean_cos[b,j] = (tr(mean_R^T M_j) - 1) / 2, the p-weighted mean of cos(angle
+    between R_n and mean_R) over the slot.  centers [B,k,3,3], 1 <= k <= 32.  NaN moments, mean_R and mean_cos for a
+    slot that holds no probability (an empty centre, all -inf scores, or exp((s - max)/T) underflowing in double) and
+    for a pair with a NaN or +inf score.  Deterministic, bit-identical whatever the batch around a pair."""
+    s, R, per_pair, c = _posterior_args(scores, R, centers)
+    B, N = s.shape
+    k = 0 if c is None else c.shape[1]
+    if k == 0:
+        raise ValueError("posterior_moments needs centers [B,k,3,3] with k >= 1")
+    f32 = dict(device=s.device, dtype=torch.float32)
+    log_z, mass, mean_cos = torch.empty(B, **f32), torch.empty(B, k, **f32), torch.empty(B, k, **f32)
+    mean_R, moment = torch.empty(B, k, 3, 3, **f32), torch.empty(B, k, 3, 3, **f32)
+    workspace, ws_bytes = _workspace(workspace, posterior_moments_workspace_bytes(B, N, k), s.device)
+    _call("ahv_posterior_moments", s.device, s.data_ptr(), R.data_ptr(), int(per_pair), c.data_ptr(), B, N, k,
+          float(radius_deg), float(temperature), log_z.data_ptr(), mass.data_ptr(), mean_R.data_ptr(), mean_cos.data_ptr(),
+          moment.data_ptr(), workspace.data_ptr(), ws_bytes)
+    return log_z, mass, mean_R, mean_cos, moment
 
 
 def topk_merge(vals: torch.Tensor, idx: torch.Tensor):

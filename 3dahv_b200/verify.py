@@ -50,6 +50,17 @@ class Posterior:
     mass: torch.Tensor                    # [B,k] probability held by each selected rotation's neighbourhood
     log_z: torch.Tensor                   # [B] log Z_b
     log_density: torch.Tensor | None      # [B,Q] log-density of R_query w.r.t. the normalised Haar measure
+    mean_R: torch.Tensor | None = None    # [B,k,3,3] p-weighted mean rotation of each slot (moments=True)
+    mean_cos: torch.Tensor | None = None  # [B,k] p-weighted mean of cos(angle to mean_R) over each slot
+    moment: torch.Tensor | None = None    # [B,k,3,3] p-weighted mean of the slot's hypothesis matrices
+
+    @property
+    def spread_deg(self) -> torch.Tensor | None:
+        """[B,k] arccos of mean_cos in degrees: each mode's width, close to the RMS angle to mean_R when the mode is
+        concentrated (None without moments)."""
+        if self.mean_cos is None:
+            return None
+        return torch.rad2deg(torch.arccos(self.mean_cos.clamp(-1.0, 1.0)))
 
 
 def _posterior_radius(min_sep_deg: float, radius_deg: float | None) -> float:
@@ -60,19 +71,24 @@ def _posterior_radius(min_sep_deg: float, radius_deg: float | None) -> float:
     return min_sep_deg
 
 
-def _posterior(scores, R, k, min_sep_deg, radius_deg, temperature, s_query) -> Posterior:
-    """The selection (`ops.topk` or `ops.topk_distinct`) and `ops.posterior_mass` over a whole [B,N] score matrix."""
+def _posterior(scores, R, k, min_sep_deg, radius_deg, temperature, s_query, moments=False) -> Posterior:
+    """The selection (`ops.topk` or `ops.topk_distinct`) and `ops.posterior_mass` (with moments: `ops.posterior_moments`)
+    over a whole [B,N] score matrix."""
     if min_sep_deg > 0:
         val, idx, R_best = ops.topk_distinct(scores, R, k, min_sep_deg)
     else:
         val, idx = ops.topk(scores, k)
         R_best = ops.gather_rotations(R, idx)
-    log_z, mass = ops.posterior_mass(scores, R, R_best, radius_deg, temperature)
+    mean_R = mean_cos = moment = None
+    if moments:
+        log_z, mass, mean_R, mean_cos, moment = ops.posterior_moments(scores, R, R_best, radius_deg, temperature)
+    else:
+        log_z, mass = ops.posterior_mass(scores, R, R_best, radius_deg, temperature)
     log_density = None
     if s_query is not None:
         N = scores.shape[1]
         log_density = (s_query.double() / temperature - log_z.double()[:, None] + math.log(N)).float()
-    return Posterior(val, idx, R_best, mass, log_z, log_density)
+    return Posterior(val, idx, R_best, mass, log_z, log_density, mean_R, mean_cos, moment)
 
 
 class HypothesisVerifier:
@@ -142,7 +158,7 @@ class HypothesisVerifier:
 
     @torch.no_grad()
     def posterior(self, vol_src, vol_tgt, R, k: int = 1, min_sep_deg: float = 0.0, radius_deg: float | None = None,
-                  temperature: float = 0.1, R_query=None) -> Posterior:
+                  temperature: float = 0.1, R_query=None, moments: bool = False) -> Posterior:
         """The selection of `score` (the top-k, or with min_sep_deg > 0 the top-k of distinct rotations) and how much of
         the verifier's softmax p_b(n) = exp(s[b,n]/T) / Z_b over the set it holds.  T = 0.1 is the InfoNCE training
         temperature (modules/model.py:43-63), under which p_b is the model's own estimate of where the rotation lies.
@@ -153,6 +169,8 @@ class HypothesisVerifier:
         `R_query` [B,Q,3,3] (e.g. the ground truth as Q = 1): `log_density` [B,Q] = s_q/T - log Z_b + log N, the
         log-density of p_b at R_query w.r.t. the normalised Haar measure (SO(3) has volume 1), meaningful when the set
         is Haar-random or near-uniform.  Subtract log(pi^2) for the convention that takes the volume of SO(3) as pi^2.
+        `moments=True` also fills `mean_R`, `mean_cos` and `moment` (`ops.posterior_moments`: the p-weighted mean
+        rotation of each slot and the mean cosine of the angle to it; `spread_deg` is its arccos in degrees).
         vol_src/vol_tgt [B,16,8,8,8]; R [N,3,3] shared or [B,N,3,3] per pair.  No host synchronisation."""
         radius_deg = _posterior_radius(min_sep_deg, radius_deg)
         dev = vol_src.device
@@ -166,7 +184,7 @@ class HypothesisVerifier:
         s_query = None
         if R_query is not None:
             s_query = ops.score(vs, tf, R_query, W1, W2, b2, k=0, math=self.math)[0]
-        return _posterior(scores, R, k, min_sep_deg, radius_deg, temperature, s_query)
+        return _posterior(scores, R, k, min_sep_deg, radius_deg, temperature, s_query, moments)
 
     @torch.no_grad()
     def predict(self, vol_src, vol_tgt, R):

@@ -350,6 +350,30 @@ AHV_API int ahv_posterior_mass(const float* scores, const float* R, int r_per_pa
                                int k, float radius_deg, float temperature, float* log_z, float* mass, void* workspace,
                                size_t workspace_bytes, void* stream);
 
+/* First moment of the posterior over each slot (extension): where inside each selected mode the probability sits, and
+ * how wide the mode is.  Slots, temperature, value rules and summation order are ahv_posterior_mass's; with
+ * e_n = exp((s[b,n] - m)/T) and W_j = sum_{n -> j} e_n (the sum mass[b,j] is formed from):
+ *   moment[b,j]   = M_j = sum_{n -> j} e_n R_n / W_j                       (3x3, row-major)
+ *   mean_R[b,j]   = argmax_{R in SO(3)} tr(R^T M_j), a proper rotation (det +1); any maximiser where it is not unique
+ *   mean_cos[b,j] = (tr(mean_R^T M_j) - 1) / 2 = E_j[cos theta(R_n, mean_R)], clamped to [-1, 1] (the hypotheses'
+ *                   fp32 matrices are orthonormal only to rounding); arccos(mean_cos) is close to the RMS angle to
+ *                   mean_R when the mode is concentrated
+ *   log_z, mass   = bit for bit ahv_posterior_mass's on the same arguments.
+ * A pair with a NaN or +inf score gets NaN everywhere.  A slot with W_j == 0 in double gets NaN moment, mean_R and
+ * mean_cos: an empty (NaN) centre, a slot whose scores are all -inf, or exp((s - m)/T) underflowing, i.e.
+ * (m - s)/T > ~745 for every hypothesis of the slot (with scores in [-1, 1] that needs T < 2.7e-3).  Sums run in
+ * double: each thread's hypotheses in index order, the warp butterfly, the warps in order, the chunks of 2048 in a
+ * fixed order; M_j is projected in double (q-method, cyclic Jacobi) and every output is cast to fp32 once, so
+ * the bits depend on the pair's inputs alone (not on B, the pair's place in the batch or the SM count).  Arguments as
+ * ahv_posterior_mass, except 1 <= k <= 32 and every output required for B > 0: mean_R and moment [B,k,3,3], mean_cos
+ * [B,k].  Two launches, workspace ahv_posterior_moments_workspace_bytes(B, N, k) (the mass's plus
+ * B * ceil(N/2048) * k * 72 bytes), no allocation, no host synchronisation: CUDA-graph capturable. */
+AHV_API size_t ahv_posterior_moments_workspace_bytes(int B, int64_t N, int k);
+AHV_API int ahv_posterior_moments(const float* scores, const float* R, int r_per_pair, const float* centers, int B,
+                                  int64_t N, int k, float radius_deg, float temperature, float* log_z, float* mass,
+                                  float* mean_R, float* mean_cos, float* moment, void* workspace,
+                                  size_t workspace_bytes, void* stream);
+
 /* torch.max / top-k over an existing score matrix (modules/model.py:195). */
 AHV_API int ahv_topk(const float* scores, int B, int64_t N, int k, int64_t idx_offset, float* topk_val,
              int64_t* topk_idx, void* workspace, size_t workspace_bytes, void* stream);

@@ -96,17 +96,19 @@ class EstimatorBase(_Base):
 
     @torch.no_grad()
     def predict_distribution(self, img_feat_src, img_feat_tgt, sampled_R=None, k: int = 1, min_sep_deg: float = 0.0,
-                             gt_R=None):
+                             gt_R=None, moments: bool = False):
         """`predict_rotation`'s selection (with min_sep_deg > 0: the top-k of rotations pairwise more than min_sep_deg
         apart) and the probability the model gives it: `HypothesisVerifier.posterior` at the training temperature
         T = 0.1 with radius cfg["DATA"]["ACC_THR"], so `mass[b,0]` is the model's estimate that pair b's prediction is
         correct at ACC_THR.  gt_R [B,3,3]: `log_density` [B,1] is the log-density of the ground-truth rotation (w.r.t.
-        the normalised Haar measure; the set should be Haar-random or near-uniform).  Returns (Posterior, sampled_R)."""
+        the normalised Haar measure; the set should be Haar-random or near-uniform).  moments=True: also each slot's
+        mean rotation `mean_R` and spread (`spread_deg`).  Returns (Posterior, sampled_R)."""
         if sampled_R is None:
             sampled_R = _ahv().so3.random_rotations(self.num_rota, device=img_feat_src.device)
         R_query = None if gt_R is None else gt_R.reshape(-1, 1, 3, 3).float().contiguous()
         post = self.verifier().posterior(img_feat_src, img_feat_tgt, sampled_R, k=k, min_sep_deg=min_sep_deg,
-                                         radius_deg=float(self.cfg["DATA"]["ACC_THR"]), temperature=0.1, R_query=R_query)
+                                         radius_deg=float(self.cfg["DATA"]["ACC_THR"]), temperature=0.1, R_query=R_query,
+                                         moments=moments)
         return post, sampled_R
 
     @torch.no_grad()
