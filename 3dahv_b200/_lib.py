@@ -25,6 +25,8 @@ SIGNATURES = {
     "ahv_so3_from_normals": (_i, [_vp, _vp, _i64, _vp]),
     "ahv_so3_sample": (_i, [_u64, _i64, _vp, _i64, _vp]),
     "ahv_so3_grid": (_i, [_i64, _i64, _vp, _i64, _vp]),
+    "ahv_so3_hopf_grid": (_i, [_i, _i64, _vp, _i64, _vp]),
+    "ahv_so3_hopf_children": (_i, [_i, _vp, _i64, _vp, _vp, _vp]),
     "ahv_so3_perturb": (_i, [_vp, _i64, _i, ctypes.c_float, _u64, _vp, _vp]),
     "ahv_rotate_volume": (_i, [_vp, _i, _vp, _vp, _vp, _i64, _vp]),
     "ahv_rotate_volume_backward": (_i, [_vp, _i, _vp, _vp, _vp, _i64, _vp]),
@@ -53,6 +55,9 @@ SIGNATURES = {
                                  _vp, _vp, _i, _i64, _i, _vp, _sz, _vp]),
     "ahv_refine_gradient_distinct": (_i, [_vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, ctypes.c_float, ctypes.c_float, _vp,
                                           _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _vp, _sz, _vp]),
+    "ahv_search_hierarchical_workspace_bytes": (_sz, [_i, _i, _i]),
+    "ahv_search_hierarchical": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp,
+                                     _sz, _vp]),
     "ahv_topk_distinct": (_i, [_vp, _vp, _i, _i, _i64, _i, ctypes.c_float, _vp, _vp, _vp, _vp]),
     "ahv_posterior_mass_workspace_bytes": (_sz, [_i, _i64, _i]),
     "ahv_posterior_mass": (_i, [_vp, _vp, _i, _vp, _i, _i64, _i, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp, _sz, _vp]),

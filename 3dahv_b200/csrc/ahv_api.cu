@@ -130,6 +130,23 @@ AHV_API int ahv_so3_grid(int64_t n_total, int64_t first_index, float* R, int64_t
   return launch_so3_grid(n_total, first_index, R, count, (cudaStream_t)stream);
 }
 
+AHV_API int ahv_so3_hopf_grid(int level, int64_t first_index, float* R, int64_t count, void* stream) {
+  if (level < 0 || level > kHopfMaxLevel || first_index < 0 || count < 0) return AHV_EINVAL;
+  if (first_index > hopf_cells(level) - count || (count > 0 && !R)) return AHV_EINVAL;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  return launch_so3_hopf_grid(level, first_index, R, count, (cudaStream_t)stream);
+}
+
+AHV_API int ahv_so3_hopf_children(int level, const int64_t* parent_idx, int64_t n, int64_t* child_idx, float* R_child,
+                                  void* stream) {
+  if (level < 0 || level >= kHopfMaxLevel || n < 0 || n > INT64_MAX / 8) return AHV_EINVAL;
+  if (n > 0 && !all_set(parent_idx, child_idx, R_child)) return AHV_EINVAL;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  return launch_so3_hopf_children(level, parent_idx, n, child_idx, R_child, (cudaStream_t)stream);
+}
+
 AHV_API int ahv_so3_perturb(const float* R_center, int64_t n, int m, float max_angle_deg, uint64_t seed, float* R_out,
                             void* stream) {
   if (n < 0 || m < 1 || !(max_angle_deg >= 0.0f) || max_angle_deg > 180.0f || (n > 0 && (!R_center || !R_out))) return AHV_EINVAL;
@@ -511,6 +528,82 @@ AHV_API int ahv_refine_gradient_distinct(const void* vol_src, int vol_dtype, con
   return refine_gradient(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, min_sep_deg,
                          first_val, first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode,
                          workspace, workspace_bytes, stream);
+}
+
+// ---- coarse-to-fine search on the nested Hopf grid (extension) --------------------------------------------
+namespace {
+constexpr int kHopfMaxBaseLevel = 6;
+
+// ahv_search_hierarchical: [scoring workspace of the larger pass | target features B*32*64 fp32 | base grid n0*9 fp32
+//  | children [B,8k] int64 | their rotations [B,8k,9] fp32 | a level's top-k [B,k] fp32 and int64 | parents [B,k] int64]
+struct HierWs {
+  size_t tgt, grid, kids, kids_R, lval, lidx, par, total;
+  HierWs(int B, int base_level, int k)
+      : tgt(std::max(VerifyWs(B, hopf_cells(base_level), k).lists, VerifyWs(B, 8 * (int64_t)k, k).lists)),
+        grid(tgt + align_up((size_t)B * kO * kP * sizeof(float), 256)),
+        kids(grid + align_up((size_t)hopf_cells(base_level) * 9 * sizeof(float), 256)),
+        kids_R(kids + align_up((size_t)B * 8 * k * sizeof(int64_t), 256)),
+        lval(kids_R + align_up((size_t)B * 8 * k * 9 * sizeof(float), 256)),
+        lidx(lval + align_up((size_t)B * k * sizeof(float), 256)),
+        par(lidx + align_up((size_t)B * k * sizeof(int64_t), 256)),
+        total(par + align_up((size_t)B * k * sizeof(int64_t), 256)) {}
+};
+}  // namespace
+
+AHV_API size_t ahv_search_hierarchical_workspace_bytes(int B, int base_level, int k) {
+  return B < 1 || base_level < 0 || base_level > kHopfMaxBaseLevel || !k_ok(k) ? 0 : HierWs(B, base_level, k).total;
+}
+
+AHV_API int ahv_search_hierarchical(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* W1, const float* W2,
+                                    const float* b2, const float* base, int base_level, int levels, int k, float* first_val,
+                                    int64_t* first_idx, float* first_R, float* val, int64_t* idx, float* R_out, int B,
+                                    int math_mode, void* workspace, size_t workspace_bytes, void* stream) {
+  if (B < 1 || !k_ok(k) || !vol_dtype_ok(vol_dtype) || !math_mode_ok(math_mode)) return AHV_EINVAL;
+  if (base_level < 0 || base_level > kHopfMaxBaseLevel || levels < 0 || base_level + levels > kHopfMaxLevel) return AHV_EINVAL;
+  if (!all_set(vol_src, vol_tgt, W1, W2, b2, base, first_val, first_idx, first_R, val, idx, R_out, workspace))
+    return AHV_EINVAL;
+  if (!all_aligned16(vol_src, vol_tgt, W1, W2, first_R, R_out, workspace)) return AHV_EINVAL;
+  const HierWs w(B, base_level, k);
+  if (workspace_bytes < w.total) return AHV_EWORKSPACE;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  cudaStream_t s = (cudaStream_t)stream;
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  float* tgt = reinterpret_cast<float*>(ws + w.tgt);
+  float* grid = reinterpret_cast<float*>(ws + w.grid);
+  int64_t* kids = reinterpret_cast<int64_t*>(ws + w.kids);
+  float* kids_R = reinterpret_cast<float*>(ws + w.kids_R);
+  int64_t* lidx = reinterpret_cast<int64_t*>(ws + w.lidx);
+  int64_t* par = reinterpret_cast<int64_t*>(ws + w.par);
+  const int64_t n0 = hopf_cells(base_level), nc = 8 * (int64_t)k;
+  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
+  if (st == AHV_OK) st = launch_so3_hopf_grid(base_level, 0, grid, n0, s);
+  // the base level: one set shared by the B pairs; its local indices are grid indices
+  if (st == AHV_OK)
+    st = ahv_score(vol_src, vol_dtype, tgt, grid, 0, W1, W2, b2, base, nullptr, first_val, first_idx, k, 0, B, n0, math_mode, ws,
+                   w.tgt, stream);
+  if (st == AHV_OK) st = launch_gather_rotations(grid, 0, first_idx, 0, B, n0, k, first_R, s);
+  if (st != AHV_OK) return st;
+  if (levels == 0) {
+    AHV_CUDA_OK(cudaMemcpyAsync(val, first_val, (size_t)B * k * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    AHV_CUDA_OK(cudaMemcpyAsync(idx, first_idx, (size_t)B * k * sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
+    AHV_CUDA_OK(cudaMemcpyAsync(R_out, first_R, (size_t)B * k * 9 * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    return AHV_OK;
+  }
+  // Each level scores the 8 children of the pair's k cells, the cells taken in ascending index order.  The candidate
+  // list then ascends in grid index (the children of cell i are 8i .. 8i+7), so the top-k's tie rule (lowest local
+  // index) is the lowest grid index.
+  st = launch_hopf_pick(nullptr, 0, first_idx, B, k, true, par, s);
+  for (int l = 0; l < levels && st == AHV_OK; ++l) {
+    const bool last = l == levels - 1;
+    st = launch_so3_hopf_children(base_level + l, par, (int64_t)B * k, kids, kids_R, s);
+    if (st == AHV_OK)
+      st = ahv_score(vol_src, vol_dtype, tgt, kids_R, 1, W1, W2, b2, base, nullptr,
+                     last ? val : reinterpret_cast<float*>(ws + w.lval), lidx, k, 0, B, nc, math_mode, ws, w.tgt, stream);
+    if (st == AHV_OK) st = launch_hopf_pick(kids, nc, lidx, B, k, !last, last ? idx : par, s);
+  }
+  if (st != AHV_OK) return st;
+  return launch_gather_rotations(kids_R, 1, lidx, 0, B, nc, k, R_out, s);
 }
 
 // ---- top-k of distinct rotations: greedy geodesic non-maximum suppression on SO(3) (extension) ------------

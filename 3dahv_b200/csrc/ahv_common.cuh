@@ -134,6 +134,15 @@ namespace peer { struct Args; }  // ahv_peer.cuh
 int launch_so3_from_normals(const float* normals, float* R, int64_t n, cudaStream_t s);
 int launch_so3_sample(uint64_t seed, int64_t first, float* R, int64_t n, cudaStream_t s);
 int launch_so3_grid(int64_t n_total, int64_t first, float* R, int64_t count, cudaStream_t s);
+// The nested Hopf x HEALPix grid (ahv_so3.cu): 72 * 8^level cells at level 0..kHopfMaxLevel.
+constexpr int kHopfMaxLevel = 16;
+__host__ __device__ constexpr int64_t hopf_cells(int level) { return (int64_t)72 << (3 * level); }
+int launch_so3_hopf_grid(int level, int64_t first, float* R, int64_t count, cudaStream_t s);
+int launch_so3_hopf_children(int level, const int64_t* parent, int64_t n, int64_t* child, float* R, cudaStream_t s);
+// Per pair, the k cells out[b,j] = cand[b, pick[b,j]] (cand NULL: pick[b,j] itself; -1 for a pick outside [0,n)), in
+// pick's order or, with `sort`, in ascending index order.  k <= 32.
+int launch_hopf_pick(const int64_t* cand, int64_t n, const int64_t* pick, int B, int k, bool sort, int64_t* out,
+                     cudaStream_t s);
 int launch_so3_perturb(const float* centers, int64_t n, int m, float max_angle_deg, uint64_t seed, float* out,
                        cudaStream_t s);
 int launch_rotate_volume(const float* vol, int per_rot, const float* R, const float* base,

@@ -7,6 +7,8 @@
 // oracle/ahv_oracle.c:ahv_oracle_so3_from_normals.
 //
 // ahv_so3_sample: native counter-based sampler (extension, SURVEY.md §8f-4).
+#include <algorithm>
+
 #include "ahv_common.cuh"
 
 namespace ahv {
@@ -105,6 +107,117 @@ __global__ void __launch_bounds__(256) so3_grid_kernel(int64_t n_total, int64_t 
   for (int e = 0; e < 9; ++e) R[t * 9 + e] = m[e];
 }
 
+// Nested, equal-volume SO(3) grid: the Hopf fibration with HEALPix on S^2 in NESTED order and a regular grid on S^1
+// (Yershova et al. 2010).  Level L: Nside = 2^L, 12*4^L pixels p, 6*2^L psi-intervals j with centres
+// psi_j = 2*pi*(j + 1/2) / (6*2^L), 72*8^L cells.  Cell i = 6*p0 + j0 at level 0; the children of cell i are 8i + 2a + b,
+// with a the HEALPix nested child digit (p' = 4p + a) and b the psi digit (j' = 2j + b), so they lie inside it.  Point:
+// (theta, phi) = the HEALPix nested pix2ang centre of p (Gorski et al. 2005) and
+// q = (cos(theta/2) cos(psi/2), cos(theta/2) sin(psi/2), sin(theta/2) cos(phi + psi/2), sin(theta/2) sin(phi + psi/2)),
+// in fp64, rounded once to fp32, then the same quaternion -> matrix map as the other generators.  Restated in numpy
+// (tests/hopf_oracle.py) and plain C (tests/hopf_oracle.c).
+__device__ __forceinline__ int64_t even_bits(uint64_t x) {  // bits 0, 2, 4, ... of x, packed
+  x &= 0x5555555555555555ull;
+  x = (x | (x >> 1)) & 0x3333333333333333ull;
+  x = (x | (x >> 2)) & 0x0f0f0f0f0f0f0f0full;
+  x = (x | (x >> 4)) & 0x00ff00ff00ff00ffull;
+  x = (x | (x >> 8)) & 0x0000ffff0000ffffull;
+  x = (x | (x >> 16)) & 0x00000000ffffffffull;
+  return (int64_t)x;
+}
+
+__device__ void hopf_rotation(int level, int64_t index, float* __restrict__ m) {
+  int64_t p = (index >> (3 * level)) / 6, j = (index >> (3 * level)) % 6;
+  for (int l = level - 1; l >= 0; --l) {
+    const int d = (int)(index >> (3 * l)) & 7;
+    p = 4 * p + (d >> 1);
+    j = 2 * j + (d & 1);
+  }
+  // pix2ang, nested: face, then the bits of the in-face index de-interleaved, then the cap and equatorial formulas
+  const int64_t nside = (int64_t)1 << level, npface = nside * nside;
+  const int face = (int)(p >> (2 * level));
+  const int64_t ipf = p & (npface - 1), ix = even_bits((uint64_t)ipf), iy = even_bits((uint64_t)ipf >> 1);
+  const int64_t jr = (int64_t)(face / 4 + 2) * nside - ix - iy - 1;  // ring number, 1 .. 4*nside - 1
+  const int jpll = 2 * (face % 4) + (face / 4 != 1);                  // 1 3 5 7 | 0 2 4 6 | 1 3 5 7
+  int64_t nr;
+  double c2, s2;  // cos^2(theta/2) = (1 + z)/2, sin^2(theta/2) = (1 - z)/2
+  if (jr < nside) {
+    nr = jr;
+    const double t = (double)(nr * nr) / (3.0 * (double)npface);  // 1 - z
+    s2 = 0.5 * t;
+    c2 = 1.0 - 0.5 * t;
+  } else if (jr > 3 * nside) {
+    nr = 4 * nside - jr;
+    const double t = (double)(nr * nr) / (3.0 * (double)npface);  // 1 + z
+    c2 = 0.5 * t;
+    s2 = 1.0 - 0.5 * t;
+  } else {
+    nr = nside;
+    const double hz = (double)(2 * nside - jr) / (3.0 * (double)nside);  // z / 2
+    c2 = 0.5 + hz;
+    s2 = 0.5 - hz;
+  }
+  int64_t tp = jpll * nr + ix - iy;  // phi = pi * tp / (4 nr)
+  if (tp < 0) tp += 8 * nr;
+  const double h = (double)(2 * j + 1) / (3.0 * (double)(nside << 2));  // psi / 2 in units of pi
+  double a = (double)tp / (4.0 * (double)nr) + h;                         // phi + psi / 2 in units of pi
+  if (a >= 2.0) a -= 2.0;
+  const double c = sqrt(c2), s = sqrt(s2);
+  double sh, ch, sa, ca;
+  sincospi(h, &sh, &ch);
+  sincospi(a, &sa, &ca);
+  quat_to_matrix_exact((float)(c * ch), (float)(c * sh), (float)(s * ca), (float)(s * sa), m);
+}
+
+__global__ void __launch_bounds__(256) so3_hopf_grid_kernel(int level, int64_t first, float* __restrict__ R, int64_t count) {
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < count; t += (int64_t)gridDim.x * blockDim.x) {
+    float m[9];
+    hopf_rotation(level, first + t, m);
+#pragma unroll
+    for (int e = 0; e < 9; ++e) R[t * 9 + e] = m[e];
+  }
+}
+
+// child t of parent t/8: index 8 * parent + t % 8 at level + 1; a parent outside the level gives -1 and NaN
+__global__ void __launch_bounds__(256) so3_hopf_children_kernel(int level, const int64_t* __restrict__ parent, int64_t n,
+                                                                int64_t* __restrict__ child, float* __restrict__ R) {
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < 8 * n; t += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t p = __ldg(parent + (t >> 3));
+    float m[9];
+    if (p >= 0 && p < hopf_cells(level)) {
+      child[t] = 8 * p + (t & 7);
+      hopf_rotation(level + 1, 8 * p + (t & 7), m);
+    } else {
+      child[t] = -1;
+#pragma unroll
+      for (int e = 0; e < 9; ++e) m[e] = __int_as_float(0x7fffffff);
+    }
+#pragma unroll
+    for (int e = 0; e < 9; ++e) R[t * 9 + e] = m[e];
+  }
+}
+
+// one warp per pair; the cells of a pair are distinct, so the rank of each among them is its sorted position
+__global__ void __launch_bounds__(128) hopf_pick_kernel(const int64_t* __restrict__ cand, int64_t n,
+                                                        const int64_t* __restrict__ pick, int B, int k, bool sort,
+                                                        int64_t* __restrict__ out) {
+  const int b = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (b >= B) return;
+  int64_t v = -1;
+  if (lane < k) {
+    v = pick[(int64_t)b * k + lane];
+    if (cand) v = (v >= 0 && v < n) ? cand[(int64_t)b * n + v] : -1;
+  }
+  int pos = lane;
+  if (sort) {
+    pos = 0;
+    for (int i = 0; i < k; ++i) {
+      const int64_t u = __shfl_sync(0xffffffffu, v, i);
+      pos += (u < v) || (u == v && i < lane);
+    }
+  }
+  if (lane < k) out[(int64_t)b * k + pos] = v;
+}
+
 // Local refinement set around given rotations (extension, BASELINE config 4 "top-k refinement pass"; the
 // reference has no refinement): out[i,0] = center[i]; out[i,j>0] = dR(i,j) @ center[i] where dR is a Haar
 // rotation (Philox counter i*m+j, same normal -> quaternion map as the sampler) whose rotation ANGLE theta in
@@ -161,6 +274,32 @@ int launch_so3_perturb(const float* centers, int64_t n, int m, float max_angle_d
 int launch_so3_grid(int64_t n_total, int64_t first, float* R, int64_t count, cudaStream_t s) {
   if (count == 0) return AHV_OK;
   so3_grid_kernel<<<(unsigned)((count + 255) / 256), 256, 0, s>>>(n_total, first, R, count);
+  AHV_CUDA_OK(cudaGetLastError());
+  return AHV_OK;
+}
+
+namespace {
+unsigned stride_blocks(int64_t items) { return (unsigned)std::min<int64_t>((items + 255) / 256, 1 << 16); }
+}  // namespace
+
+int launch_so3_hopf_grid(int level, int64_t first, float* R, int64_t count, cudaStream_t s) {
+  if (count == 0) return AHV_OK;
+  so3_hopf_grid_kernel<<<stride_blocks(count), 256, 0, s>>>(level, first, R, count);
+  AHV_CUDA_OK(cudaGetLastError());
+  return AHV_OK;
+}
+
+int launch_so3_hopf_children(int level, const int64_t* parent, int64_t n, int64_t* child, float* R, cudaStream_t s) {
+  if (n == 0) return AHV_OK;
+  so3_hopf_children_kernel<<<stride_blocks(8 * n), 256, 0, s>>>(level, parent, n, child, R);
+  AHV_CUDA_OK(cudaGetLastError());
+  return AHV_OK;
+}
+
+int launch_hopf_pick(const int64_t* cand, int64_t n, const int64_t* pick, int B, int k, bool sort, int64_t* out,
+                     cudaStream_t s) {
+  if (B == 0) return AHV_OK;
+  hopf_pick_kernel<<<(unsigned)((B + 3) / 4), 128, 0, s>>>(cand, n, pick, B, k, sort, out);
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }

@@ -106,6 +106,69 @@ def grid_rotations(n_total: int, first_index: int = 0, count: int | None = None,
     return R
 
 
+HOPF_MAX_LEVEL, HOPF_MAX_BASE_LEVEL = 16, 6
+
+
+def hopf_cells(level: int) -> int:
+    """Cells of level `level` of the nested Hopf grid: 72 * 8^level."""
+    return 72 * 8 ** level
+
+
+def hopf_grid(level: int, first_index: int = 0, count: int | None = None, device="cuda") -> torch.Tensor:
+    """ahv_so3_hopf_grid: cells [first_index, first_index + count) of level `level` (0..16) of the nested, equal-volume
+    Hopf x HEALPix SO(3) grid, as rotations [count,3,3] (cell i's children at level + 1 are 8i .. 8i+7)."""
+    count = hopf_cells(level) - first_index if count is None else count
+    R = torch.empty(count, 3, 3, device=torch.device(device), dtype=torch.float32)
+    _call("ahv_so3_hopf_grid", R.device, int(level), int(first_index), R.data_ptr(), int(count))
+    return R
+
+
+def hopf_children(level: int, parent_idx: torch.Tensor):
+    """ahv_so3_hopf_children: cells parent_idx [...] of level `level` (0..15) -> their 8 children at level + 1 in child
+    order, (child_idx [...,8] int64, R [...,8,3,3]); bit for bit `hopf_grid(level + 1)` at child_idx.  A parent outside the
+    level gives children -1 with NaN rotations."""
+    p = _dev(parent_idx, "parent_idx", torch.int64)
+    n = p.numel()
+    child = torch.empty(*p.shape, 8, device=p.device, dtype=torch.int64)
+    R = torch.empty(*p.shape, 8, 3, 3, device=p.device, dtype=torch.float32)
+    _call("ahv_so3_hopf_children", p.device, int(level), p.data_ptr(), n, child.data_ptr(), R.data_ptr())
+    return child, R
+
+
+def search_hierarchical_workspace_bytes(B: int, base_level: int, k: int) -> int:
+    """Bytes of scratch `search_hierarchical` needs (0 for invalid sizes); it holds the base grid, 36 B per cell."""
+    return int(_lib.lib().ahv_search_hierarchical_workspace_bytes(B, base_level, k))
+
+
+def search_hierarchical(vol_src, vol_tgt, W1, W2, b2, base_level: int = 2, levels: int = 4, k: int = 8, math: int = MATH_TC,
+                        workspace: torch.Tensor | None = None, out=None):
+    """ahv_search_hierarchical: coarse-to-fine search on the nested Hopf grid in one C call - the whole base level scored
+    and cut to its top-k, then `levels` times the 8 children of each pair's k cells scored and cut to their top-k.  No
+    torch ops, no host synchronisation, CUDA-graph capturable (pass `out` = the tuple a previous call returned to reuse
+    its buffers).  Returns (first_val [B,k], first_idx [B,k], first_R [B,k,3,3] - the base level's top-k, indices of
+    level base_level - val [B,k], idx [B,k], R [B,k,3,3] - the finest level's top-k, indices of level
+    base_level + levels; slot 0 is the answer - workspace)."""
+    vs, vdt = _vol_src(vol_src)
+    vt = _dev(vol_tgt, "vol_tgt")
+    B = vs.shape[0]
+    if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
+        raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
+    if not (1 <= k <= 32 and 0 <= base_level <= HOPF_MAX_BASE_LEVEL and levels >= 0 and base_level + levels <= HOPF_MAX_LEVEL):
+        raise ValueError("1 <= k <= 32, 0 <= base_level <= 6, levels >= 0 and base_level + levels <= 16 expected")
+    W1, W2, b2 = _head(W1, W2, b2)
+    dev = vs.device
+    if out is None:
+        f = dict(device=dev, dtype=torch.float32)
+        out = (torch.empty(B, k, **f), torch.empty(B, k, device=dev, dtype=torch.int64), torch.empty(B, k, 3, 3, **f),
+               torch.empty(B, k, **f), torch.empty(B, k, device=dev, dtype=torch.int64), torch.empty(B, k, 3, 3, **f))
+    fv, fi, fR, v, i, R = out[:6]
+    workspace, ws_bytes = _workspace(workspace, search_hierarchical_workspace_bytes(B, base_level, k), dev)
+    _call("ahv_search_hierarchical", dev, vs.data_ptr(), vdt, vt.data_ptr(), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
+          base_coords(dev).data_ptr(), int(base_level), int(levels), int(k), fv.data_ptr(), fi.data_ptr(), fR.data_ptr(),
+          v.data_ptr(), i.data_ptr(), R.data_ptr(), B, int(math), workspace.data_ptr(), ws_bytes)
+    return fv, fi, fR, v, i, R, workspace
+
+
 def perturb_rotations(R_center: torch.Tensor, m: int, max_angle_deg: float, seed: int = 0) -> torch.Tensor:
     """ahv_so3_perturb: [...,3,3] centres -> [...,m,3,3] rotations within `max_angle_deg` of them (index 0 = the
     centre itself)."""

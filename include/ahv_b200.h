@@ -101,6 +101,21 @@ AHV_API int ahv_so3_sample(uint64_t seed, int64_t first_index, float* R, int64_t
  * matrices.  Evaluated in fp64, rounded once: bit-identical to oracle/ahv_oracle.c. */
 AHV_API int ahv_so3_grid(int64_t n_total, int64_t first_index, float* R, int64_t count, void* stream);
 
+/* Nested, equal-volume SO(3) grid (extension): the Hopf fibration, HEALPix on S^2 in NESTED order times a regular
+ * grid on S^1 (Yershova et al. 2010).  Level L (0 <= L <= 16): Nside = 2^L, 12*4^L pixels p, 6*2^L psi-intervals j
+ * with centres psi_j = 2*pi*(j + 1/2)/(6*2^L), 72*8^L cells of equal Haar volume.  Cell index i = 6*p0 + j0 at level
+ * 0; the children of cell i at level L + 1 are 8i + 2a + b (a: the HEALPix nested child digit, p' = 4p + a; b: the
+ * psi digit, j' = 2j + b), and lie inside it.  Point: (theta, phi) = HEALPix nested pix2ang(Nside, p) and
+ * q = (cos(theta/2)cos(psi/2), cos(theta/2)sin(psi/2), sin(theta/2)cos(phi+psi/2), sin(theta/2)sin(phi+psi/2)),
+ * evaluated in fp64, rounded once to fp32, then ahv_so3_from_normals' quaternion -> matrix map.
+ * ahv_so3_hopf_grid: cells [first_index, first_index + count) of `level` as rotation matrices R [count,3,3]. */
+AHV_API int ahv_so3_hopf_grid(int level, int64_t first_index, float* R, int64_t count, void* stream);
+/* For each of the n cells parent_idx[i] of `level` (0 <= level < 16), its 8 children at level + 1 in child order:
+ * child_idx [n,8] (= 8*parent_idx[i] + c) and R_child [n,8,3,3], bit-identical to ahv_so3_hopf_grid(level + 1) at
+ * those indices.  A parent index outside [0, 72*8^level) gives children -1 with NaN rotations. */
+AHV_API int ahv_so3_hopf_children(int level, const int64_t* parent_idx, int64_t n, int64_t* child_idx, float* R_child,
+                                  void* stream);
+
 /* Local refinement set (extension, BASELINE config 4 "top-k refinement pass"; the reference has none):
  * R_out[i,0] = R_center[i]; R_out[i,j] = dR(i,j) @ R_center[i] for 0 < j < m, dR a Haar rotation (Philox
  * counter i*m+j keyed by seed) whose angle is rescaled from [0,pi] to [0,max_angle_deg] about its axis.
@@ -316,6 +331,25 @@ AHV_API int ahv_refine_gradient_distinct(const void* vol_src, int vol_dtype, con
                                          int64_t* first_idx, float* first_R, float* R_all, float* score_all, float* best_val,
                                          int64_t* best_idx, float* R_best, int B, int64_t N, int math_mode, void* workspace,
                                          size_t workspace_bytes, void* stream);
+
+/* Coarse-to-fine search on the nested Hopf grid (extension; see ahv_so3_hopf_grid), one call:
+ *   target features once (ahv_forward_3d2d); the whole grid of base_level (72*8^base_level cells, shared by the B
+ *   pairs) is generated into the workspace and scored with ahv_score(math_mode), its top-k in first_val [B,k],
+ *   first_idx [B,k] (grid indices of base_level) and first_R [B,k,3,3];
+ *   then `levels` times: the 8 children of each pair's k cells, the cells taken in ascending index order, form a
+ *   per-pair set [B,8k] (ascending grid indices of the next level), scored with ahv_score(math_mode) and cut to its
+ *   top-k, whose cells are the next parents.
+ * val [B,k], idx [B,k] (grid indices of level base_level + levels) and R_out [B,k,3,3] (= ahv_so3_hopf_grid of that
+ * level at idx) are the top-k of the finest level, in ahv_topk's order: slot 0 is the answer, ties go to the lowest
+ * index.  levels = 0 gives the base level's top-k.  0 <= base_level <= 6, base_level + levels <= 16, 1 <= k <= 32,
+ * B >= 1; every buffer required, rotation buffers, volumes, W1, W2 and the workspace 16-byte aligned.  Workspace:
+ * ahv_search_hierarchical_workspace_bytes(B, base_level, k) (0 for invalid sizes), which holds the base grid
+ * (36 B * 72*8^base_level).  No allocation, no host synchronisation: CUDA-graph capturable. */
+AHV_API size_t ahv_search_hierarchical_workspace_bytes(int B, int base_level, int k);
+AHV_API int ahv_search_hierarchical(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* W1, const float* W2,
+                                    const float* b2, const float* base, int base_level, int levels, int k, float* first_val,
+                                    int64_t* first_idx, float* first_R, float* val, int64_t* idx, float* R_out, int B,
+                                    int math_mode, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Top-k of distinct rotations (extension): greedy geodesic non-maximum suppression on SO(3) over the score-sorted
  * hypotheses of each pair.  With key(n) = ahv_topk's order (score descending, ties -> lowest index, NaN as ahv_topk
