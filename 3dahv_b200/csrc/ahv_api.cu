@@ -51,24 +51,16 @@ struct RefineWs {
       : cand(VerifyWs(B, N, k).total), total(cand + VerifyWs(B, (int64_t)k * m, 1).total) {}
 };
 
-// ahv_refine_gradient: [the grid pass's verification workspace | target features B*32*64 fp32 | top-k partials over [B,k]]
-struct RefineGradientWs {
-  size_t tgt, top, total;
-  RefineGradientWs(int B, int64_t N, int k)
-      : tgt(VerifyWs(B, N, k).total),
-        top(tgt + align_up((size_t)B * kO * kP * sizeof(float), 256)),
-        total(top + align_up(topk_workspace_bytes(B, k, 1), 256)) {}
-};
-
-// ahv_refine_gradient_sharded (world > 1), per = ceil(N / world) hypotheses at most on a rank:
-// [the slice's verification workspace | the slice's rotations B*per*9 | the whole score matrix B*N (distinct pass 1)
-//  | target features B*32*64 | top-k partials over [B,k]]
+// ahv_refine_gradient(_distinct) (world == 1) and ahv_refine_gradient_sharded, per = ceil(N / world) hypotheses at most
+// on a rank: [the slice's verification workspace | the slice's rotations B*per*9 | the whole score matrix B*N (distinct
+// pass 1) | target features B*32*64 | top-k partials over [B,k]].  One GPU scores R in place and keeps the distinct
+// pass's scores in the verification workspace, so its two middle regions are empty.
 struct ShardedRefineWs {
   size_t rs, full, tgt, top, total;
   ShardedRefineWs(int B, int64_t N, int k, int world)
       : rs(VerifyWs(B, (N + world - 1) / world, k).total),
-        full(rs + align_up((size_t)B * (size_t)((N + world - 1) / world) * 9 * sizeof(float), 256)),
-        tgt(full + align_up((size_t)B * (size_t)N * sizeof(float), 256)),
+        full(rs + (world > 1 ? align_up((size_t)B * (size_t)((N + world - 1) / world) * 9 * sizeof(float), 256) : 0)),
+        tgt(full + (world > 1 ? align_up((size_t)B * (size_t)N * sizeof(float), 256) : 0)),
         top(tgt + align_up((size_t)B * kO * kP * sizeof(float), 256)),
         total(top + align_up(topk_workspace_bytes(B, k, 1), 256)) {}
 };
@@ -89,6 +81,150 @@ void shard_bounds(int64_t n, int rank, int world, int64_t* lo, int64_t* hi) {
   const int64_t per = (n + world - 1) / world;
   *lo = std::min(n, (int64_t)rank * per);
   *hi = std::min(n, *lo + per);
+}
+
+// ---- chains: the device work of the entries, once their arguments have been checked -------------------------------
+// Each entry checks its arguments, then the device, then composes chains and launch_* functions; no entry calls
+// another (the host-buffer entries aside).  `pa` == nullptr or a group of one is one GPU.
+
+// ahv_score: the scores (into `scores`, else the workspace's score region) and, for k > 0, their top-k
+int score_chain(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R, int r_per_pair, const float* W1,
+                const float* W2, const float* b2, const float* base, float* scores, float* topk_val, int64_t* topk_idx, int k,
+                int64_t idx_offset, int B, int64_t N, int math_mode, unsigned char* ws, cudaStream_t s) {
+  const VerifyWs w(B, N, k);
+  float* sc = scores ? scores : reinterpret_cast<float*>(ws);
+  int st;
+  if (math_mode == AHV_MATH_FP32)
+    st = launch_score_fp32(vol_src, vol_dtype, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, sc, B, N, s);
+  else
+    st = launch_score_tc(vol_src, vol_dtype, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, sc, B, N, ws + w.tc,
+                         w.lists - w.tc, s, math_mode == AHV_MATH_TC_F16GATHER);
+  if (st != AHV_OK) return st;
+  if (k > 0) st = launch_topk(sc, B, N, k, idx_offset, topk_val, topk_idx, ws + w.topk, w.tc - w.topk, s);
+  return st;
+}
+
+// ahv_verify (B*N > 0) and a shard's step of ahv_verify_sharded (N == 0: an empty shard, which still joins the exchange).
+// The fused launchers get the caller's scratch from the tensor-core region on: its end on one GPU, `lists` on a shard,
+// whose per-shard lists follow.  A shard returns the whole set's selection only, so it passes no scores.
+int verify_chain(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair, const float* W1,
+                 const float* W2, const float* b2, const float* base, float* scores, float* topk_val, int64_t* topk_idx,
+                 float* R_best, int k, int64_t idx_offset, int B, int64_t N, int math_mode, void* workspace,
+                 size_t workspace_bytes, cudaStream_t s, const peer::Args* pa) {
+  if (pa && pa->world == 1) pa = nullptr;
+  const VerifyWs w(B, N, k);
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  const size_t tc_bytes = pa ? w.lists - w.tc : workspace_bytes - w.tc;  // packed weights, target features, scales, keys
+  if (N > 0 && screened(w, vol_dtype, math_mode, scores, k, B, N))  // a shard's last pass exchanges and merges the winners
+    return launch_verify_tc_screened(static_cast<const float*>(vol_src), vol_tgt, R, r_per_pair != 0, W1, W2, b2, base,
+                                     topk_val, topk_idx, R_best, idx_offset, B, N, ws + w.tc, tc_bytes,
+                                     reinterpret_cast<float*>(ws), ws + w.topk, s, pa);
+  // three launches, nothing but 40 B per hypothesis touches HBM; a shard's scoring kernel exchanges and merges itself
+  if (N > 0 && k == 1 && math_mode != AHV_MATH_FP32)
+    return launch_verify_tc_argmax(vol_src, vol_dtype, vol_tgt, R, r_per_pair != 0, W1, W2, b2, base, scores, topk_val,
+                                   topk_idx, R_best, idx_offset, B, N, ws + w.tc, tc_bytes, s,
+                                   math_mode == AHV_MATH_TC_F16GATHER, pa);
+  float* tgt = scratch_tgt_feat(ws + w.tc, B);
+  int st;
+  if (!pa) {  // target features, scores and top-k, winner gather
+    st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
+    if (st != AHV_OK) return st;
+    st = score_chain(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, scores, topk_val, topk_idx, k, idx_offset, B,
+                     N, math_mode, ws, s);
+    if (st != AHV_OK || !R_best) return st;
+    return launch_gather_rotations(R, r_per_pair != 0, topk_idx, idx_offset, B, N, k, R_best, s);
+  }
+  // a shard with k > 1 (or empty, or fp32 FFMA arithmetic): its local top-k, then the exchange kernel
+  float* l_val = reinterpret_cast<float*>(ws + w.lists);
+  int64_t* l_idx = reinterpret_cast<int64_t*>(ws + w.lists + align_up((size_t)B * k * sizeof(float), 8));
+  const int kl = N < k ? (int)N : k;
+  if (kl < k) {  // pad with (-inf, -1), which the merge ignores
+    AHV_CUDA_OK(cudaMemsetAsync(l_val, 0xff, (size_t)B * k * sizeof(float), s));
+    AHV_CUDA_OK(cudaMemsetAsync(l_idx, 0xff, (size_t)B * k * sizeof(int64_t), s));
+  }
+  if (N > 0) {
+    st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
+    if (st != AHV_OK) return st;
+    if (kl == k) {
+      st = score_chain(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, nullptr, l_val, l_idx, k, idx_offset, B, N,
+                       math_mode, ws, s);
+    } else {  // fewer hypotheses than k on this shard: compact [B,kl] lists (in the output buffers, which the
+              // exchange overwrites afterwards), then spread into the padded [B,k]
+      st = score_chain(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, nullptr, topk_val, topk_idx, kl, idx_offset,
+                       B, N, math_mode, ws, s);
+      if (st != AHV_OK) return st;
+      AHV_CUDA_OK(cudaMemcpy2DAsync(l_val, (size_t)k * sizeof(float), topk_val, (size_t)kl * sizeof(float),
+                                    (size_t)kl * sizeof(float), B, cudaMemcpyDeviceToDevice, s));
+      AHV_CUDA_OK(cudaMemcpy2DAsync(l_idx, (size_t)k * sizeof(int64_t), topk_idx, (size_t)kl * sizeof(int64_t),
+                                    (size_t)kl * sizeof(int64_t), B, cudaMemcpyDeviceToDevice, s));
+    }
+    if (st != AHV_OK) return st;
+  }
+  return launch_topk_exchange(l_val, l_idx, R, r_per_pair != 0, idx_offset, N, B, k, topk_val, topk_idx, R_best, *pa, s);
+}
+
+// ahv_refine_gradient(_distinct) and ahv_refine_gradient_sharded: the first pass (top-k, or with min_sep_deg > 0 the
+// distinct top-k of every score), target features, gradient ascent of each winner, per-pair arg-max.  A rank of a group
+// scores its shard_bounds slice of R, exchanges the first pass, ascends its share of the B*k slots and gathers every
+// ascended slot; every rank then holds the whole-set result.
+int refine_gradient_chain(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
+                          const float* W1, const float* W2, const float* b2, const float* base, int k, int steps,
+                          float step_deg, float min_sep_deg, float* first_val, int64_t* first_idx, float* first_R,
+                          float* R_all, float* score_all, float* best_val, int64_t* best_idx, float* R_best, int B, int64_t N,
+                          int math_mode, void* workspace, cudaStream_t s, const peer::Args* pa, int64_t peer_max_hyps) {
+  if (pa && pa->world == 1) pa = nullptr;
+  const ShardedRefineWs w(B, N, k, pa ? pa->world : 1);
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  float* tgt = reinterpret_cast<float*>(ws + w.tgt);
+  const bool distinct = min_sep_deg > 0.0f;
+  int64_t lo = 0, hi = N;
+  if (pa) shard_bounds(N, pa->rank, pa->world, &lo, &hi);
+  const int64_t n = hi - lo;
+  const float* rs = pa ? reinterpret_cast<float*>(ws + w.rs) : R;
+  if (pa && n > 0)  // this rank's rotations, 16-byte aligned for the scorers (a shared set: one row)
+    AHV_CUDA_OK(cudaMemcpy2DAsync(ws + w.rs, (size_t)n * 9 * sizeof(float), R + (size_t)lo * 9, (size_t)N * 9 * sizeof(float),
+                                  (size_t)n * 9 * sizeof(float), r_per_pair ? B : 1, cudaMemcpyDeviceToDevice, s));
+  int st;
+  if (!distinct) {
+    // pass 1: the top-k and their rotations (a shard's, exchanged and merged into the whole set's)
+    st = verify_chain(vol_src, vol_dtype, vol_tgt, rs, r_per_pair, W1, W2, b2, base, nullptr, first_val, first_idx, first_R, k,
+                      lo, B, n, math_mode, ws, w.rs, s, pa);
+    if (st != AHV_OK) return st;
+  }
+  // the ascent scores in fp32 against fp32 target features (bit-equal to ahv_forward_3d2d), whatever math_mode is
+  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
+  if (st != AHV_OK) return st;
+  if (distinct) {
+    // pass 1: every score of the set (the fused k = 1 arg-max writes none), a shard's all-gathered into the whole [B,N]
+    // on every rank, then the k distinct winners: the SAME greedy selection over the whole set on every rank (per-shard
+    // NMS lists do not merge into the global one)
+    const float* sc = reinterpret_cast<const float*>(ws);
+    if (n > 0) {
+      st = score_chain(vol_src, vol_dtype, tgt, rs, r_per_pair, W1, W2, b2, base, nullptr, nullptr, nullptr, 0, 0, B, n,
+                       math_mode, ws, s);
+      if (st != AHV_OK) return st;
+    }
+    if (pa) {
+      float* full = reinterpret_cast<float*>(ws + w.full);
+      st = launch_scores_exchange(sc, B, N, full, *pa, peer_max_hyps, s);
+      if (st != AHV_OK) return st;
+      sc = full;
+    }
+    st = launch_topk_distinct(sc, R, r_per_pair != 0, B, N, k, min_sep_deg, first_val, first_idx, first_R, s);
+    if (st != AHV_OK) return st;
+  }
+  // empty slots (fewer than k distinct winners) are not ascended: R_all NaN, score_all -inf.  One GPU ascends every
+  // slot (item_hi < 0), a rank its share, after which every ascended slot goes to every rank.
+  int64_t ilo = 0, ihi = -1;
+  if (pa) shard_bounds((int64_t)B * k, pa->rank, pa->world, &ilo, &ihi);
+  st = launch_gradient_ascent(vol_src, vol_dtype, tgt, first_R, W1, W2, b2, base, steps, step_deg, R_all, score_all, B, k, s,
+                              distinct ? first_idx : nullptr, ilo, ihi);
+  if (st == AHV_OK && pa) st = launch_slot_gather(R_all, score_all, ilo, ihi, B, k, *pa, s);
+  if (st != AHV_OK) return st;
+  // per-pair arg-max over the k ascended candidates (on every rank)
+  st = launch_topk(score_all, B, k, 1, 0, best_val, best_idx, ws + w.top, w.total - w.top, s);
+  if (st != AHV_OK || !R_best) return st;
+  return launch_gather_rotations(R_all, 1, best_idx, 0, B, k, 1, R_best, s);
 }
 
 }  // namespace
@@ -354,22 +490,9 @@ AHV_API int ahv_score(const void* vol_src, int vol_dtype, const float* tgt_feat,
   int st = check_device();
   if (st != AHV_OK) return st;
   if ((int64_t)B * N == 0) return AHV_OK;
-
-  const VerifyWs w(B, N, k);
-  if (!workspace || workspace_bytes < w.lists) return AHV_EWORKSPACE;
-  unsigned char* ws = static_cast<unsigned char*>(workspace);
-  float* sc = scores ? scores : reinterpret_cast<float*>(ws);
-
-  cudaStream_t s = (cudaStream_t)stream;
-  if (math_mode == AHV_MATH_FP32)
-    st = launch_score_fp32(vol_src, vol_dtype, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, sc, B,
-                           N, s);
-  else
-    st = launch_score_tc(vol_src, vol_dtype, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, sc, B, N,
-                         ws + w.tc, w.lists - w.tc, s, math_mode == AHV_MATH_TC_F16GATHER);
-  if (st != AHV_OK) return st;
-  if (k > 0) st = launch_topk(sc, B, N, k, idx_offset, topk_val, topk_idx, ws + w.topk, w.tc - w.topk, s);
-  return st;
+  if (!workspace || workspace_bytes < VerifyWs(B, N, k).lists) return AHV_EWORKSPACE;
+  return score_chain(vol_src, vol_dtype, tgt_feat, R, r_per_pair, W1, W2, b2, base, scores, topk_val, topk_idx, k, idx_offset,
+                     B, N, math_mode, static_cast<unsigned char*>(workspace), (cudaStream_t)stream);
 }
 
 AHV_API int ahv_verify(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
@@ -382,27 +505,9 @@ AHV_API int ahv_verify(const void* vol_src, int vol_dtype, const float* vol_tgt,
   int st = check_device();
   if (st != AHV_OK) return st;
   if ((int64_t)B * N == 0) return AHV_OK;
-  const VerifyWs w(B, N, k);
-  if (!workspace || workspace_bytes < w.total) return AHV_EWORKSPACE;
-  cudaStream_t s = (cudaStream_t)stream;
-  void* ws_tc = static_cast<unsigned char*>(workspace) + w.tc;  // packed weights, target features, scales, keys
-  if (screened(w, vol_dtype, math_mode, scores, k, B, N))
-    return launch_verify_tc_screened(static_cast<const float*>(vol_src), vol_tgt, R, r_per_pair != 0, W1, W2, b2, base,
-                                     topk_val, topk_idx, R_best, idx_offset, B, N, ws_tc, workspace_bytes - w.tc,
-                                     static_cast<float*>(workspace), static_cast<unsigned char*>(workspace) + w.topk, s);
-  if (math_mode != AHV_MATH_FP32 && k == 1)  // three launches, nothing but 40 B per hypothesis touches HBM
-    return launch_verify_tc_argmax(vol_src, vol_dtype, vol_tgt, R, r_per_pair != 0, W1, W2, b2, base, scores,
-                                   topk_val, topk_idx, R_best, idx_offset, B, N, ws_tc,
-                                   workspace_bytes - w.tc, s, math_mode == AHV_MATH_TC_F16GATHER);
-  float* tgt = scratch_tgt_feat(ws_tc, B);
-  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
-  if (st != AHV_OK) return st;
-  st = ahv_score(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, scores, topk_val, topk_idx, k,
-                 idx_offset, B, N, math_mode, workspace, workspace_bytes, stream);
-  if (st != AHV_OK) return st;
-  if (R_best)
-    st = launch_gather_rotations(R, r_per_pair != 0, topk_idx, idx_offset, B, N, k, R_best, s);
-  return st;
+  if (!workspace || workspace_bytes < VerifyWs(B, N, k).total) return AHV_EWORKSPACE;
+  return verify_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, scores, topk_val, topk_idx, R_best, k,
+                      idx_offset, B, N, math_mode, workspace, workspace_bytes, (cudaStream_t)stream, nullptr);
 }
 
 // ---- two-pass selection: dense set -> top-k -> local refinement (BASELINE config 4; extension) -----------
@@ -420,17 +525,24 @@ AHV_API int ahv_refine(const void* vol_src, int vol_dtype, const float* vol_tgt,
   if (!aligned16(cand)) return AHV_EINVAL;
   const RefineWs w(B, N, k, m);
   if (workspace_bytes < w.total) return AHV_EWORKSPACE;
+  if (!n_ok(N) || !vol_dtype_ok(vol_dtype) || !math_mode_ok(math_mode)) return AHV_EINVAL;
+  if (!all_set(vol_src, vol_tgt, R, W1, W2, b2, base)) return AHV_EINVAL;
+  if (!all_aligned16(vol_src, vol_tgt, R, W1, W2, workspace)) return AHV_EINVAL;
+  if (!(max_angle_deg >= 0.0f) || max_angle_deg > 180.0f) return AHV_EINVAL;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  cudaStream_t s = (cudaStream_t)stream;
   unsigned char* ws = static_cast<unsigned char*>(workspace);
   // pass 1: the whole set, top-k and their rotations
-  int st = ahv_verify(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, first_val, first_idx, first_R, k,
-                      0, B, N, math_mode, ws, w.cand, stream);
+  st = verify_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, first_val, first_idx, first_R, k, 0,
+                    B, N, math_mode, ws, w.cand, s, nullptr);
   if (st != AHV_OK) return st;
   // candidates: m rotations within max_angle_deg of each of the B*k winners (index 0 = the winner itself)
-  st = ahv_so3_perturb(first_R, (int64_t)B * k, m, max_angle_deg, seed, cand, stream);
+  st = launch_so3_perturb(first_R, (int64_t)B * k, m, max_angle_deg, seed, cand, s);
   if (st != AHV_OK) return st;
   // pass 2: per-pair candidate sets [B, k*m], arg-max
-  return ahv_verify(vol_src, vol_dtype, vol_tgt, cand, 1, W1, W2, b2, base, nullptr, best_val, best_idx, R_best, 1, 0, B,
-                    (int64_t)k * m, math_mode, ws + w.cand, w.total - w.cand, stream);
+  return verify_chain(vol_src, vol_dtype, vol_tgt, cand, 1, W1, W2, b2, base, nullptr, best_val, best_idx, R_best, 1, 0, B,
+                      (int64_t)k * m, math_mode, ws + w.cand, w.total - w.cand, s, nullptr);
 }
 
 // ---- gradient ascent of the fp32 score on SO(3), alone and after the grid pass (extension) ---------------
@@ -454,58 +566,23 @@ AHV_API int ahv_gradient_ascent(const void* vol_src, int vol_dtype, const float*
 }
 
 AHV_API size_t ahv_refine_gradient_workspace_bytes(int B, int64_t N, int k) {
-  return B < 0 || N < 0 || !k_ok(k) ? 0 : RefineGradientWs(B, N, k).total;
+  return B < 0 || N < 0 || !k_ok(k) ? 0 : ShardedRefineWs(B, N, k, 1).total;
 }
 
 namespace {
 bool min_sep_ok(float min_sep_deg) { return std::isfinite(min_sep_deg) && min_sep_deg >= 0.0f && min_sep_deg <= 180.0f; }
 
-// ahv_refine_gradient (min_sep_deg == 0) and ahv_refine_gradient_distinct: the same chain apart from its first pass
-int refine_gradient(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair, const float* W1,
-                    const float* W2, const float* b2, const float* base, int k, int steps, float step_deg, float min_sep_deg,
-                    float* first_val, int64_t* first_idx, float* first_R, float* R_all, float* score_all, float* best_val,
-                    int64_t* best_idx, float* R_best, int B, int64_t N, int math_mode, void* workspace,
-                    size_t workspace_bytes, void* stream) {
-  if (B < 1 || N < 1 || !n_ok(N) || !k_ok(k) || k > N) return AHV_EINVAL;
-  if (!ascent_args_ok(vol_dtype, steps, step_deg) || !min_sep_ok(min_sep_deg) || !math_mode_ok(math_mode)) return AHV_EINVAL;
-  if (!all_set(vol_src, vol_tgt, R, W1, W2, b2, base, first_val, first_idx, first_R, R_all, score_all, best_val, best_idx,
-               workspace))
-    return AHV_EINVAL;
-  if (!all_aligned16(vol_src, vol_tgt, R, W1, W2, first_R, R_all, R_best, workspace)) return AHV_EINVAL;
-  const RefineGradientWs w(B, N, k);
-  if (workspace_bytes < w.total) return AHV_EWORKSPACE;
-  int st = check_device();
-  if (st != AHV_OK) return st;
-  cudaStream_t s = (cudaStream_t)stream;
-  unsigned char* ws = static_cast<unsigned char*>(workspace);
-  float* tgt = reinterpret_cast<float*>(ws + w.tgt);
-  const bool distinct = min_sep_deg > 0.0f;
-  if (!distinct) {
-    // pass 1: the whole set, top-k and their rotations
-    st = ahv_verify(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, first_val, first_idx, first_R, k,
-                    0, B, N, math_mode, ws, w.tgt, stream);
-    if (st != AHV_OK) return st;
-  }
-  // the ascent scores in fp32 against fp32 target features (bit-equal to ahv_forward_3d2d), whatever math_mode is
-  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
-  if (st != AHV_OK) return st;
-  if (distinct) {
-    // pass 1: every score of the set (the fused k = 1 arg-max writes none), then the k distinct winners
-    st = ahv_score(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, nullptr, nullptr, nullptr, 0, 0, B, N,
-                   math_mode, ws, w.tgt, stream);
-    if (st != AHV_OK) return st;
-    st = launch_topk_distinct(reinterpret_cast<const float*>(ws), R, r_per_pair != 0, B, N, k, min_sep_deg, first_val,
-                              first_idx, first_R, s);
-    if (st != AHV_OK) return st;
-  }
-  // empty slots (fewer than k distinct winners) are not ascended: R_all NaN, score_all -inf
-  st = launch_gradient_ascent(vol_src, vol_dtype, tgt, first_R, W1, W2, b2, base, steps, step_deg, R_all, score_all, B, k, s,
-                              distinct ? first_idx : nullptr);
-  if (st != AHV_OK) return st;
-  // per-pair arg-max over the k ascended candidates
-  st = launch_topk(score_all, B, k, 1, 0, best_val, best_idx, ws + w.top, w.total - w.top, s);
-  if (st != AHV_OK || !R_best) return st;
-  return launch_gather_rotations(R_all, 1, best_idx, 0, B, k, 1, R_best, s);
+// the argument rules of the gradient-refinement entries (min_sep_deg == 0: ahv_refine_gradient's plain top-k)
+bool refine_gradient_args_ok(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, const float* W1,
+                             const float* W2, const float* b2, const float* base, int k, int steps, float step_deg,
+                             float min_sep_deg, const float* first_val, const int64_t* first_idx, const float* first_R,
+                             const float* R_all, const float* score_all, const float* best_val, const int64_t* best_idx,
+                             const float* R_best, int B, int64_t N, int math_mode, const void* workspace) {
+  if (B < 1 || N < 1 || !n_ok(N) || !k_ok(k) || k > N) return false;
+  if (!ascent_args_ok(vol_dtype, steps, step_deg) || !min_sep_ok(min_sep_deg) || !math_mode_ok(math_mode)) return false;
+  return all_set(vol_src, vol_tgt, R, W1, W2, b2, base, first_val, first_idx, first_R, R_all, score_all, best_val, best_idx,
+                 workspace) &&
+         all_aligned16(vol_src, vol_tgt, R, W1, W2, first_R, R_all, R_best, workspace);
 }
 }  // namespace
 
@@ -514,9 +591,15 @@ AHV_API int ahv_refine_gradient(const void* vol_src, int vol_dtype, const float*
                                 float step_deg, float* first_val, int64_t* first_idx, float* first_R, float* R_all,
                                 float* score_all, float* best_val, int64_t* best_idx, float* R_best, int B, int64_t N,
                                 int math_mode, void* workspace, size_t workspace_bytes, void* stream) {
-  return refine_gradient(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, 0.0f, first_val,
-                         first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode, workspace,
-                         workspace_bytes, stream);
+  if (!refine_gradient_args_ok(vol_src, vol_dtype, vol_tgt, R, W1, W2, b2, base, k, steps, step_deg, 0.0f, first_val, first_idx,
+                               first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode, workspace))
+    return AHV_EINVAL;
+  if (workspace_bytes < ShardedRefineWs(B, N, k, 1).total) return AHV_EWORKSPACE;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  return refine_gradient_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, 0.0f, first_val,
+                               first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode, workspace,
+                               (cudaStream_t)stream, nullptr, 0);
 }
 
 AHV_API int ahv_refine_gradient_distinct(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R,
@@ -525,9 +608,15 @@ AHV_API int ahv_refine_gradient_distinct(const void* vol_src, int vol_dtype, con
                                          int64_t* first_idx, float* first_R, float* R_all, float* score_all, float* best_val,
                                          int64_t* best_idx, float* R_best, int B, int64_t N, int math_mode, void* workspace,
                                          size_t workspace_bytes, void* stream) {
-  return refine_gradient(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, min_sep_deg,
-                         first_val, first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode,
-                         workspace, workspace_bytes, stream);
+  if (!refine_gradient_args_ok(vol_src, vol_dtype, vol_tgt, R, W1, W2, b2, base, k, steps, step_deg, min_sep_deg, first_val,
+                               first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode, workspace))
+    return AHV_EINVAL;
+  if (workspace_bytes < ShardedRefineWs(B, N, k, 1).total) return AHV_EWORKSPACE;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  return refine_gradient_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, min_sep_deg,
+                               first_val, first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode,
+                               workspace, (cudaStream_t)stream, nullptr, 0);
 }
 
 // ---- coarse-to-fine search on the nested Hopf grid (extension) --------------------------------------------
@@ -580,8 +669,8 @@ AHV_API int ahv_search_hierarchical(const void* vol_src, int vol_dtype, const fl
   if (st == AHV_OK) st = launch_so3_hopf_grid(base_level, 0, grid, n0, s);
   // the base level: one set shared by the B pairs; its local indices are grid indices
   if (st == AHV_OK)
-    st = ahv_score(vol_src, vol_dtype, tgt, grid, 0, W1, W2, b2, base, nullptr, first_val, first_idx, k, 0, B, n0, math_mode, ws,
-                   w.tgt, stream);
+    st = score_chain(vol_src, vol_dtype, tgt, grid, 0, W1, W2, b2, base, nullptr, first_val, first_idx, k, 0, B, n0, math_mode, ws,
+                     s);
   if (st == AHV_OK) st = launch_gather_rotations(grid, 0, first_idx, 0, B, n0, k, first_R, s);
   if (st != AHV_OK) return st;
   if (levels == 0) {
@@ -598,8 +687,8 @@ AHV_API int ahv_search_hierarchical(const void* vol_src, int vol_dtype, const fl
     const bool last = l == levels - 1;
     st = launch_so3_hopf_children(base_level + l, par, (int64_t)B * k, kids, kids_R, s);
     if (st == AHV_OK)
-      st = ahv_score(vol_src, vol_dtype, tgt, kids_R, 1, W1, W2, b2, base, nullptr,
-                     last ? val : reinterpret_cast<float*>(ws + w.lval), lidx, k, 0, B, nc, math_mode, ws, w.tgt, stream);
+      st = score_chain(vol_src, vol_dtype, tgt, kids_R, 1, W1, W2, b2, base, nullptr,
+                       last ? val : reinterpret_cast<float*>(ws + w.lval), lidx, k, 0, B, nc, math_mode, ws, s);
     if (st == AHV_OK) st = launch_hopf_pick(kids, nc, lidx, B, k, !last, last ? idx : par, s);
   }
   if (st != AHV_OK) return st;
@@ -794,50 +883,10 @@ AHV_API int ahv_verify_sharded(const void* vol_src, int vol_dtype, const float* 
   if (world > 1 && (B > peer_max_pairs || k > peer_max_k)) return AHV_EINVAL;  // exchange buffer too small for this call
   st = check_device();
   if (st != AHV_OK) return st;
-  if (world == 1)
-    return N == 0 ? AHV_EINVAL
-                  : ahv_verify(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, topk_val, topk_idx,
-                               R_best, k, idx_offset, B, N, math_mode, workspace, workspace_bytes, stream);
-  const VerifyWs w(B, N, k);
-  if (!workspace || workspace_bytes < w.total) return AHV_EWORKSPACE;
-  unsigned char* ws = static_cast<unsigned char*>(workspace);
-  cudaStream_t s = (cudaStream_t)stream;
-  if (N > 0 && screened(w, vol_dtype, math_mode, nullptr, k, B, N))  // its last pass exchanges and merges the winners
-    return launch_verify_tc_screened(static_cast<const float*>(vol_src), vol_tgt, R, r_per_pair != 0, W1, W2, b2, base,
-                                     topk_val, topk_idx, R_best, idx_offset, B, N, ws + w.tc, w.lists - w.tc,
-                                     reinterpret_cast<float*>(ws), ws + w.topk, s, &pa);
-  if (k == 1 && N > 0 && math_mode != AHV_MATH_FP32)  // the scoring kernel exchanges and merges the winners itself
-    return launch_verify_tc_argmax(vol_src, vol_dtype, vol_tgt, R, r_per_pair != 0, W1, W2, b2, base, nullptr, topk_val,
-                                   topk_idx, R_best, idx_offset, B, N, ws + w.tc, w.lists - w.tc, s,
-                                   math_mode == AHV_MATH_TC_F16GATHER, &pa);
-  // k > 1 (or an empty shard, or fp32 FFMA arithmetic): local top-k of the shard, then the exchange kernel
-  float* l_val = reinterpret_cast<float*>(ws + w.lists);
-  int64_t* l_idx = reinterpret_cast<int64_t*>(ws + w.lists + align_up((size_t)B * k * sizeof(float), 8));
-  const int kl = N < k ? (int)N : k;
-  if (kl < k) {  // pad with (-inf, -1), which the merge ignores
-    AHV_CUDA_OK(cudaMemsetAsync(l_val, 0xff, (size_t)B * k * sizeof(float), s));
-    AHV_CUDA_OK(cudaMemsetAsync(l_idx, 0xff, (size_t)B * k * sizeof(int64_t), s));
-  }
-  if (N > 0) {
-    float* tgt = scratch_tgt_feat(ws + w.tc, B);
-    st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
-    if (st != AHV_OK) return st;
-    if (kl == k) {
-      st = ahv_score(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, nullptr, l_val, l_idx, k, idx_offset, B, N,
-                     math_mode, workspace, workspace_bytes, stream);
-    } else {  // fewer hypotheses than k on this shard: compact [B,kl] lists (in the output buffers, which the
-              // exchange overwrites afterwards), then spread into the padded [B,k]
-      st = ahv_score(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, nullptr, topk_val, topk_idx, kl, idx_offset, B,
-                     N, math_mode, workspace, workspace_bytes, stream);
-      if (st != AHV_OK) return st;
-      AHV_CUDA_OK(cudaMemcpy2DAsync(l_val, (size_t)k * sizeof(float), topk_val, (size_t)kl * sizeof(float),
-                                    (size_t)kl * sizeof(float), B, cudaMemcpyDeviceToDevice, s));
-      AHV_CUDA_OK(cudaMemcpy2DAsync(l_idx, (size_t)k * sizeof(int64_t), topk_idx, (size_t)kl * sizeof(int64_t),
-                                    (size_t)kl * sizeof(int64_t), B, cudaMemcpyDeviceToDevice, s));
-    }
-    if (st != AHV_OK) return st;
-  }
-  return launch_topk_exchange(l_val, l_idx, R, r_per_pair != 0, idx_offset, N, B, k, topk_val, topk_idx, R_best, pa, s);
+  if (world == 1 && N == 0) return AHV_EINVAL;
+  if (!workspace || workspace_bytes < VerifyWs(B, N, k).total) return AHV_EWORKSPACE;
+  return verify_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, topk_val, topk_idx, R_best, k,
+                      idx_offset, B, N, math_mode, workspace, workspace_bytes, (cudaStream_t)stream, &pa);
 }
 
 AHV_API int ahv_scores_exchange(const float* part, int B, int64_t N, float* scores, int rank, int world, void* const* peers,
@@ -857,7 +906,7 @@ AHV_API int ahv_scores_exchange(const float* part, int B, int64_t N, float* scor
 
 AHV_API size_t ahv_refine_gradient_sharded_workspace_bytes(int B, int64_t N, int k, int world) {
   if (B < 0 || N < 0 || !k_ok(k) || world < 1 || world > peer::kMaxPeers) return 0;
-  return world == 1 ? RefineGradientWs(B, N, k).total : ShardedRefineWs(B, N, k, world).total;
+  return ShardedRefineWs(B, N, k, world).total;
 }
 
 AHV_API int ahv_refine_gradient_sharded(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R,
@@ -867,70 +916,20 @@ AHV_API int ahv_refine_gradient_sharded(const void* vol_src, int vol_dtype, cons
                                         int64_t* best_idx, float* R_best, int B, int64_t N, int math_mode, void* workspace,
                                         size_t workspace_bytes, int rank, int world, void* const* peers, int peer_max_pairs,
                                         int peer_max_k, int64_t peer_max_hyps, void* stream) {
-  if (B < 1 || N < 1 || !n_ok(N) || !k_ok(k) || k > N) return AHV_EINVAL;
-  if (!ascent_args_ok(vol_dtype, steps, step_deg) || !min_sep_ok(min_sep_deg) || !math_mode_ok(math_mode)) return AHV_EINVAL;
-  if (!all_set(vol_src, vol_tgt, R, W1, W2, b2, base, first_val, first_idx, first_R, R_all, score_all, best_val, best_idx,
-               workspace))
+  if (!refine_gradient_args_ok(vol_src, vol_dtype, vol_tgt, R, W1, W2, b2, base, k, steps, step_deg, min_sep_deg, first_val,
+                               first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode, workspace))
     return AHV_EINVAL;
-  if (!all_aligned16(vol_src, vol_tgt, R, W1, W2, first_R, R_all, R_best, workspace)) return AHV_EINVAL;
   peer::Args pa;
   int st = make_peer_args(rank, world, peers, peer_max_pairs, peer_max_k, &pa);
   if (st != AHV_OK) return st;
-  const bool distinct = min_sep_deg > 0.0f;
   if (world > 1 && (B > peer_max_pairs || k > peer_max_k)) return AHV_EINVAL;  // the slot gather's entries
-  if (world > 1 && distinct && (!n_ok(peer_max_hyps) || N > peer_max_hyps)) return AHV_EINVAL;  // the score region
-  if (world == 1)
-    return refine_gradient(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, min_sep_deg,
-                           first_val, first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode,
-                           workspace, workspace_bytes, stream);
-  const ShardedRefineWs w(B, N, k, world);
-  if (workspace_bytes < w.total) return AHV_EWORKSPACE;
+  if (world > 1 && min_sep_deg > 0.0f && (!n_ok(peer_max_hyps) || N > peer_max_hyps)) return AHV_EINVAL;  // the score region
+  if (workspace_bytes < ShardedRefineWs(B, N, k, world).total) return AHV_EWORKSPACE;
   st = check_device();
   if (st != AHV_OK) return st;
-  cudaStream_t s = (cudaStream_t)stream;
-  unsigned char* ws = static_cast<unsigned char*>(workspace);
-  float* rs = reinterpret_cast<float*>(ws + w.rs);
-  float* tgt = reinterpret_cast<float*>(ws + w.tgt);
-  int64_t lo, hi;
-  shard_bounds(N, rank, world, &lo, &hi);
-  const int64_t n = hi - lo;
-  if (n > 0)  // this rank's rotations, 16-byte aligned for the scorers (a shared set: one row)
-    AHV_CUDA_OK(cudaMemcpy2DAsync(rs, (size_t)n * 9 * sizeof(float), R + (size_t)lo * 9, (size_t)N * 9 * sizeof(float),
-                                  (size_t)n * 9 * sizeof(float), r_per_pair ? B : 1, cudaMemcpyDeviceToDevice, s));
-  if (!distinct) {
-    // pass 1: the slice's top-k, exchanged and merged into the whole set's top-k with its rotations
-    st = ahv_verify_sharded(vol_src, vol_dtype, vol_tgt, rs, r_per_pair, W1, W2, b2, base, first_val, first_idx, first_R, k, lo,
-                            B, n, math_mode, ws, w.rs, rank, world, peers, peer_max_pairs, peer_max_k, stream);
-    if (st != AHV_OK) return st;
-  }
-  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
-  if (st != AHV_OK) return st;
-  if (distinct) {
-    // pass 1: the slice's scores, all-gathered into the whole [B,N] on every rank, then the SAME greedy selection
-    // over the whole set on every rank (per-shard NMS lists do not merge into the global one)
-    float* full = reinterpret_cast<float*>(ws + w.full);
-    if (n > 0) {
-      st = ahv_score(vol_src, vol_dtype, tgt, rs, r_per_pair, W1, W2, b2, base, nullptr, nullptr, nullptr, 0, 0, B, n,
-                     math_mode, ws, w.rs, stream);
-      if (st != AHV_OK) return st;
-    }
-    st = launch_scores_exchange(reinterpret_cast<const float*>(ws), B, N, full, pa, peer_max_hyps, s);
-    if (st != AHV_OK) return st;
-    st = launch_topk_distinct(full, R, r_per_pair != 0, B, N, k, min_sep_deg, first_val, first_idx, first_R, s);
-    if (st != AHV_OK) return st;
-  }
-  // this rank's share of the B*k ascents, then every ascended slot to every rank
-  int64_t ilo, ihi;
-  shard_bounds((int64_t)B * k, rank, world, &ilo, &ihi);
-  st = launch_gradient_ascent(vol_src, vol_dtype, tgt, first_R, W1, W2, b2, base, steps, step_deg, R_all, score_all, B, k, s,
-                              distinct ? first_idx : nullptr, ilo, ihi);
-  if (st != AHV_OK) return st;
-  st = launch_slot_gather(R_all, score_all, ilo, ihi, B, k, pa, s);
-  if (st != AHV_OK) return st;
-  // per-pair arg-max over the k ascended candidates, on every rank
-  st = launch_topk(score_all, B, k, 1, 0, best_val, best_idx, ws + w.top, w.total - w.top, s);
-  if (st != AHV_OK || !R_best) return st;
-  return launch_gather_rotations(R_all, 1, best_idx, 0, B, k, 1, R_best, s);
+  return refine_gradient_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, min_sep_deg,
+                               first_val, first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode,
+                               workspace, (cudaStream_t)stream, &pa, peer_max_hyps);
 }
 
 // ---- host-buffer entries -------------------------------------------------------------------------------

@@ -60,6 +60,24 @@ def _vol_src(vol_src):
     return _dev(vol_src, "vol_src"), VOL_F32
 
 
+def _vols(vol_src, vol_tgt):
+    """A source / target pair of [B,16,8,8,8] volumes: (vol_src, its AHV_VOL_* code, vol_tgt, B)."""
+    vs, vdt = _vol_src(vol_src)
+    vt = _dev(vol_tgt, "vol_tgt")
+    B = vs.shape[0]
+    if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
+        raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
+    return vs, vdt, vt, B
+
+
+def _peer_args(peer):
+    """The peer arguments of the sharded entries - rank, world, the group's exchange buffers, their capacity in pairs and
+    in k - for `peer` (a `dist.PeerExchange`), or for one GPU when it is None."""
+    if peer is None:
+        return 0, 1, None, 0, 0
+    return peer.rank, peer.world, (ctypes.c_void_p * peer.world)(*[int(p) for p in peer.ptrs]), peer.max_pairs, peer.max_k
+
+
 def _head(W1, W2, b2):
     """The verification head's weights as the kernels read them: W1 [32,384], W2 [32,32], b2 [32]."""
     return _dev(W1.reshape(32, 384), "W1"), _dev(W2.reshape(32, 32), "W2"), _dev(b2, "b2")
@@ -148,11 +166,7 @@ def search_hierarchical(vol_src, vol_tgt, W1, W2, b2, base_level: int = 2, level
     its buffers).  Returns (first_val [B,k], first_idx [B,k], first_R [B,k,3,3] - the base level's top-k, indices of
     level base_level - val [B,k], idx [B,k], R [B,k,3,3] - the finest level's top-k, indices of level
     base_level + levels; slot 0 is the answer - workspace)."""
-    vs, vdt = _vol_src(vol_src)
-    vt = _dev(vol_tgt, "vol_tgt")
-    B = vs.shape[0]
-    if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
-        raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
+    vs, vdt, vt, B = _vols(vol_src, vol_tgt)
     if not (1 <= k <= 32 and 0 <= base_level <= HOPF_MAX_BASE_LEVEL and levels >= 0 and base_level + levels <= HOPF_MAX_LEVEL):
         raise ValueError("1 <= k <= 32, 0 <= base_level <= 6, levels >= 0 and base_level + levels <= 16 expected")
     W1, W2, b2 = _head(W1, W2, b2)
@@ -415,19 +429,20 @@ def score(vol_src, tgt_feat, R, W1, W2, b2, k: int = 1, idx_offset: int = 0, mat
     return scores, val, idx
 
 
+def _verify_args(vol_src, vol_tgt, R, W1, W2, b2):
+    """The inputs of `verify` and `verify_sharded` as their entries read them: (vs, vdt, vt, R, per_pair, W1, W2, b2, B, N)."""
+    vs, vdt, vt, B = _vols(vol_src, vol_tgt)
+    R, per_pair, N = _rotations(_dev(R, "R"), B)
+    return (vs, vdt, vt, R, per_pair, *_head(W1, W2, b2), B, N)
+
+
 def verify(vol_src, vol_tgt, R, W1, W2, b2, k: int = 1, idx_offset: int = 0, math: int = MATH_TC,
            return_scores: bool = False, gather: bool = True, workspace: torch.Tensor | None = None):
     """ahv_verify: target features + fused scoring + selection + winner gather in one C call.
     Returns (scores|None, topk_val [B,k], topk_idx [B,k], R_best [B,k,3,3]|None)."""
-    vs, vdt = _vol_src(vol_src)
-    vt = _dev(vol_tgt, "vol_tgt")
-    B = vs.shape[0]
-    if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
-        raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
-    R, per_pair, N = _rotations(_dev(R, "R"), B)
+    vs, vdt, vt, R, per_pair, W1, W2, b2, B, N = _verify_args(vol_src, vol_tgt, R, W1, W2, b2)
     if k < 1 or k > 32:
         raise ValueError("k must be in [1,32]")
-    W1, W2, b2 = _head(W1, W2, b2)
     dev = vs.device
     scores = torch.empty(B, N, device=dev, dtype=torch.float32) if return_scores else None
     val = torch.empty(B, k, device=dev, dtype=torch.float32)
@@ -463,12 +478,8 @@ def refine(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, m: int = 64, max_angle_
     torch ops, CUDA-graph capturable (pass `out` = the tuple a previous call returned to reuse its buffers).
     Returns (first_val [B,k], first_idx [B,k], first_R [B,k,3,3], cand [B,k*m,3,3], best_val [B], best_idx [B],
     R_best [B,3,3], workspace)."""
-    vs, vdt = _vol_src(vol_src)
-    vt = _dev(vol_tgt, "vol_tgt")
-    B = vs.shape[0]
+    vs, vdt, vt, B = _vols(vol_src, vol_tgt)
     R, per_pair, N = _rotations(_dev(R, "R"), B)
-    if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
-        raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
     if not (1 <= k <= min(32, N)) or m < 1:
         raise ValueError("1 <= k <= min(32, N) and m >= 1 expected")
     W1, W2, b2 = _head(W1, W2, b2)
@@ -517,14 +528,19 @@ def refine_gradient(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, steps: int = 2
     its empty slots come back as first_idx -1, R_all NaN, score_all -inf.
     Returns (first_val [B,k], first_idx [B,k], first_R [B,k,3,3], R_all [B,k,3,3], score_all [B,k], best_val [B],
     best_idx [B], R_best [B,3,3], workspace)."""
-    vs, vdt = _vol_src(vol_src)
-    vt = _dev(vol_tgt, "vol_tgt")
-    B = vs.shape[0]
+    return _refine_gradient(vol_src, vol_tgt, R, W1, W2, b2, None, k, steps, step_deg, math, workspace, out, min_sep_deg)
+
+
+def _refine_gradient(vol_src, vol_tgt, R, W1, W2, b2, peer, k, steps, step_deg, math, workspace, out, min_sep_deg):
+    """`refine_gradient` (peer None) and `refine_gradient_sharded`."""
+    vs, vdt, vt, B = _vols(vol_src, vol_tgt)
     R, per_pair, N = _rotations(_dev(R, "R"), B)
-    if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
-        raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
     if not 1 <= k <= min(32, N):
         raise ValueError("1 <= k <= min(32, N) expected")
+    max_hyps = getattr(peer, "max_hyps", 0)
+    if peer is not None and peer.world > 1 and (B > peer.max_pairs or k > peer.max_k or (min_sep_deg > 0 and N > max_hyps)):
+        raise ValueError(f"exchange buffer holds {peer.max_pairs} pairs x top-{peer.max_k} x {max_hyps} scores; got B={B}, k={k}, "
+                         f"N={N}")
     W1, W2, b2 = _head(W1, W2, b2)
     dev = vs.device
     if out is None:
@@ -533,22 +549,21 @@ def refine_gradient(vol_src, vol_tgt, R, W1, W2, b2, k: int = 32, steps: int = 2
                torch.empty(B, k, 3, 3, **f), torch.empty(B, k, **f), torch.empty(B, **f),
                torch.empty(B, device=dev, dtype=torch.int64), torch.empty(B, 3, 3, **f))
     fv, fi, fR, Ra, sa, bv, bi, bR = out[:8]
-    workspace, ws_bytes = _workspace(workspace, int(_lib.lib().ahv_refine_gradient_workspace_bytes(B, N, k)), dev)
+    lib = _lib.lib()
+    need = (lib.ahv_refine_gradient_workspace_bytes(B, N, k) if peer is None
+            else lib.ahv_refine_gradient_sharded_workspace_bytes(B, N, k, peer.world))
+    workspace, ws_bytes = _workspace(workspace, int(need), dev)
     head = (vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
             base_coords(dev).data_ptr(), k, int(steps), float(step_deg))
     tail = (fv.data_ptr(), fi.data_ptr(), fR.data_ptr(), Ra.data_ptr(), sa.data_ptr(), bv.data_ptr(), bi.data_ptr(), bR.data_ptr(),
             B, N, math, workspace.data_ptr(), ws_bytes)
-    if min_sep_deg == 0:
+    if peer is not None:
+        _call("ahv_refine_gradient_sharded", dev, *head, float(min_sep_deg), *tail, *_peer_args(peer), max_hyps)
+    elif min_sep_deg == 0:
         _call("ahv_refine_gradient", dev, *head, *tail)
     else:
         _call("ahv_refine_gradient_distinct", dev, *head, float(min_sep_deg), *tail)
     return fv, fi, fR, Ra, sa, bv, bi, bR, workspace
-
-
-def _peer_array(peer):
-    import ctypes
-
-    return (ctypes.c_void_p * peer.world)(*[int(p) for p in peer.ptrs])
 
 
 def verify_sharded(vol_src, vol_tgt, R, W1, W2, b2, idx_offset: int, peer, k: int = 1, math: int = MATH_TC,
@@ -558,14 +573,7 @@ def verify_sharded(vol_src, vol_tgt, R, W1, W2, b2, idx_offset: int, peer, k: in
     them (k == 1 with tensor-core arithmetic: inside the scoring kernel; otherwise one exchange kernel after the
     shard's top-k).  Returns (topk_val [B,k], topk_idx [B,k] global, R_best [B,k,3,3]) over the whole set,
     identical on every rank.  An empty slice ([0,3,3]) is allowed."""
-    vs, vdt = _vol_src(vol_src)
-    vt = _dev(vol_tgt, "vol_tgt")
-    R = _dev(R, "R")
-    W1, W2, b2 = _head(W1, W2, b2)
-    B = vs.shape[0]
-    R, per_pair, N = _rotations(R, B)
-    if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
-        raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
+    vs, vdt, vt, R, per_pair, W1, W2, b2, B, N = _verify_args(vol_src, vol_tgt, R, W1, W2, b2)
     if B > peer.max_pairs or k > peer.max_k:
         raise ValueError(f"exchange buffer holds {peer.max_pairs} pairs x top-{peer.max_k}; got B={B}, k={k}")
     dev = vs.device
@@ -575,7 +583,7 @@ def verify_sharded(vol_src, vol_tgt, R, W1, W2, b2, idx_offset: int, peer, k: in
     workspace, ws_bytes = _workspace(workspace, workspace_bytes(B, N, k), dev)
     _call("ahv_verify_sharded", dev, vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr() if N else None, int(per_pair), W1.data_ptr(),
           W2.data_ptr(), b2.data_ptr(), base_coords(dev).data_ptr(), val.data_ptr(), idx.data_ptr(), Rb.data_ptr(), k, idx_offset,
-          B, N, math, workspace.data_ptr(), ws_bytes, peer.rank, peer.world, _peer_array(peer), peer.max_pairs, peer.max_k)
+          B, N, math, workspace.data_ptr(), ws_bytes, *_peer_args(peer))
     return val, idx, Rb
 
 
@@ -590,7 +598,7 @@ def topk_exchange(val, idx, R, idx_offset: int, peer):
     out_i = torch.empty(B, k, device=dev, dtype=torch.int64)
     Rb = torch.empty(B, k, 3, 3, device=dev, dtype=torch.float32)
     _call("ahv_topk_exchange", dev, v.data_ptr(), i.data_ptr(), R.data_ptr() if N else None, int(per_pair), idx_offset, N, B, k,
-          out_v.data_ptr(), out_i.data_ptr(), Rb.data_ptr(), peer.rank, peer.world, _peer_array(peer), peer.max_pairs, peer.max_k)
+          out_v.data_ptr(), out_i.data_ptr(), Rb.data_ptr(), *_peer_args(peer))
     return out_v, out_i, Rb
 
 
@@ -609,8 +617,7 @@ def scores_exchange(part, N: int, peer, out=None):
     if B > peer.max_pairs or N > max_hyps:
         raise ValueError(f"exchange buffer holds {peer.max_pairs} pairs x {max_hyps} scores; got B={B}, N={N}")
     out = torch.empty(B, N, device=p.device, dtype=torch.float32) if out is None else out
-    _call("ahv_scores_exchange", p.device, p.data_ptr() if hi > lo else None, B, N, out.data_ptr(), peer.rank, peer.world,
-          _peer_array(peer), peer.max_pairs, peer.max_k, max_hyps)
+    _call("ahv_scores_exchange", p.device, p.data_ptr() if hi > lo else None, B, N, out.data_ptr(), *_peer_args(peer), max_hyps)
     return out
 
 
@@ -622,34 +629,7 @@ def refine_gradient_sharded(vol_src, vol_tgt, R, W1, W2, b2, peer, k: int = 32, 
     first pass (top-k lists, or with min_sep_deg > 0 the score matrix, after which the distinct selection runs on
     every rank) and the ascended slots through NVLink peer memory.  min_sep_deg > 0 needs peer.max_hyps >= N.
     One C call, no NCCL, CUDA-graph capturable (`out` = a previous result's tuple).  Returns `refine_gradient`'s tuple."""
-    vs, vdt = _vol_src(vol_src)
-    vt = _dev(vol_tgt, "vol_tgt")
-    B = vs.shape[0]
-    R, per_pair, N = _rotations(_dev(R, "R"), B)
-    if tuple(vs.shape[1:]) != (16, 8, 8, 8) or tuple(vt.shape) != (B, 16, 8, 8, 8):
-        raise ValueError("vol_src / vol_tgt must be [B,16,8,8,8]")
-    if not 1 <= k <= min(32, N):
-        raise ValueError("1 <= k <= min(32, N) expected")
-    max_hyps = getattr(peer, "max_hyps", 0)
-    if peer.world > 1 and (B > peer.max_pairs or k > peer.max_k or (min_sep_deg > 0 and N > max_hyps)):
-        raise ValueError(f"exchange buffer holds {peer.max_pairs} pairs x top-{peer.max_k} x {max_hyps} scores; got B={B}, k={k}, "
-                         f"N={N}")
-    W1, W2, b2 = _head(W1, W2, b2)
-    dev = vs.device
-    if out is None:
-        f = dict(device=dev, dtype=torch.float32)
-        out = (torch.empty(B, k, **f), torch.empty(B, k, device=dev, dtype=torch.int64), torch.empty(B, k, 3, 3, **f),
-               torch.empty(B, k, 3, 3, **f), torch.empty(B, k, **f), torch.empty(B, **f),
-               torch.empty(B, device=dev, dtype=torch.int64), torch.empty(B, 3, 3, **f))
-    fv, fi, fR, Ra, sa, bv, bi, bR = out[:8]
-    need = int(_lib.lib().ahv_refine_gradient_sharded_workspace_bytes(B, N, k, peer.world))
-    workspace, ws_bytes = _workspace(workspace, need, dev)
-    _call("ahv_refine_gradient_sharded", dev, vs.data_ptr(), vdt, vt.data_ptr(), R.data_ptr(), int(per_pair), W1.data_ptr(),
-          W2.data_ptr(), b2.data_ptr(), base_coords(dev).data_ptr(), k, int(steps), float(step_deg), float(min_sep_deg),
-          fv.data_ptr(), fi.data_ptr(), fR.data_ptr(), Ra.data_ptr(), sa.data_ptr(), bv.data_ptr(), bi.data_ptr(), bR.data_ptr(),
-          B, N, math, workspace.data_ptr(), ws_bytes, peer.rank, peer.world, _peer_array(peer), peer.max_pairs, peer.max_k,
-          max_hyps)
-    return fv, fi, fR, Ra, sa, bv, bi, bR, workspace
+    return _refine_gradient(vol_src, vol_tgt, R, W1, W2, b2, peer, k, steps, step_deg, math, workspace, out, min_sep_deg)
 
 
 def topk(scores: torch.Tensor, k: int, idx_offset: int = 0):
@@ -776,8 +756,6 @@ class HostSession:
     """Caller-owned device scratch of the host-buffer entry (`ahv_host_session_create`), reused across calls."""
 
     def __init__(self, device="cuda"):
-        import ctypes
-
         self.device = torch.device(device)
         h = ctypes.c_void_p()
         with torch.cuda.device(self.device):
@@ -825,8 +803,7 @@ def predict_host(vol_src, vol_tgt, R, W1, W2, b2, k: int = 1, math: int = MATH_T
     try:
         _call("ahv_predict_host_ex", device, session.handle, vs.data_ptr(), VOL_BF16 if bf16 else VOL_F32, vt.data_ptr(),
               Rc.data_ptr(), int(per_pair), W1c.data_ptr(), W2c.data_ptr(), b2c.data_ptr(), base.data_ptr(), sc, val.data_ptr(),
-              idx.data_ptr(), Rb.data_ptr(), k, idx_offset, B, N, math, peer.rank if peer else 0, peer.world if peer else 1,
-              _peer_array(peer) if peer else None, peer.max_pairs if peer else 0, peer.max_k if peer else 0)
+              idx.data_ptr(), Rb.data_ptr(), k, idx_offset, B, N, math, *_peer_args(peer))
     finally:
         if own:
             session.close()

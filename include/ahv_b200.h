@@ -286,7 +286,8 @@ AHV_API int ahv_verify_screen_stats(const void* workspace, int B, int64_t N, int
  * candidates around every winner (cand [B,k*m,3,3], caller-provided, 16-byte aligned; candidate j*m is winner
  * j itself); ahv_verify over each pair's own k*m candidates keeping the best (best_val [B], best_idx [B] = index
  * into that pair's candidate set, R_best [B,3,3] or NULL).  No host synchronisation, no allocation:
- * CUDA-graph capturable.  k <= min(32, N).  Workspace: ahv_refine_workspace_bytes. */
+ * CUDA-graph capturable.  k <= min(32, N), 0 <= max_angle_deg <= 180: every argument, max_angle_deg included, is
+ * checked before the first pass is enqueued, so a rejected call writes nothing.  Workspace: ahv_refine_workspace_bytes. */
 AHV_API size_t ahv_refine_workspace_bytes(int B, int64_t N, int k, int m);
 AHV_API int ahv_refine(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
                        const float* W1, const float* W2, const float* b2, const float* base, int k, int m,

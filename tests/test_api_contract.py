@@ -206,6 +206,35 @@ def test_workspace_bounds_on_the_device(ahv):
     bounded(need, lambda ws, n: lib.ahv_refine_gradient_distinct(*head, k, 5, 1.0, 20.0, *outs, B, N, 0, ws, n, stream))
 
 
+@pytest.mark.gpu
+@pytest.mark.parametrize("max_angle_deg", (-1.0, 181.0, math.nan))
+def test_rejected_refine_leaves_its_outputs_untouched(ahv, max_angle_deg):
+    """ahv_refine checks max_angle_deg before its first pass: a rejected call enqueues no work and writes nothing."""
+    import torch
+
+    lib = ahv._lib.lib()
+    dev = torch.device("cuda", 0)
+    B, N, k, m = 2, 300, 4, 8
+    g = torch.Generator().manual_seed(7)
+    T = lambda *s: torch.randn(*s, generator=g).to(dev)
+    vs, vt = T(B, 16, 8, 8, 8), T(B, 16, 8, 8, 8)
+    R = ahv.so3.grid_rotations(N, device=dev)
+    W1, W2, b2 = T(32, 384) * 0.05, T(32, 32) * 0.2, T(32) * 0.1
+    outs = [torch.full(s, 7.0, device=dev) for s in ((B, k), (B, k, 3, 3), (B, k * m, 3, 3), (B,), (B, 3, 3))]
+    idx = [torch.full(s, 7, device=dev, dtype=torch.int64) for s in ((B, k), (B,))]
+    fv, fR, cand, bv, bR = outs
+    fi, bi = idx
+    need = lib.ahv_refine_workspace_bytes(B, N, k, m)
+    ws = torch.empty(need, device=dev, dtype=torch.uint8)
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    st = lib.ahv_refine(vs.data_ptr(), 0, vt.data_ptr(), R.data_ptr(), 0, W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
+                        ahv.ops.base_coords(dev).data_ptr(), k, m, max_angle_deg, 0, fv.data_ptr(), fi.data_ptr(), fR.data_ptr(),
+                        cand.data_ptr(), bv.data_ptr(), bi.data_ptr(), bR.data_ptr(), B, N, 0, ws.data_ptr(), need, stream)
+    torch.cuda.synchronize(dev)
+    assert st == EINVAL
+    assert all(bool((t == 7).all()) for t in outs + idx)
+
+
 # ---- frozen values ---------------------------------------------------------------------------------------------------
 SIZES = {
     'ahv_workspace_bytes': {
@@ -605,12 +634,13 @@ STATUSES = {
             'workspace_bytes=0 workspace_bytes=need-1 '),
         ECUDA: (
             'valid vol_dtype=1 math_mode=1 math_mode=2 B=1 N=2147483647 k=1 k=32 m=1 m=536870911 '
-            'max_angle_deg=-1.0 max_angle_deg=180.0 max_angle_deg=181.0 max_angle_deg=nan workspace_bytes=need '
+            'max_angle_deg=180.0 workspace_bytes=need '
             'b2=20 b2=24 base=20 base=24 first_val=20 first_val=24 first_idx=20 first_idx=24 first_R=20 '
             'first_R=24 best_val=20 best_val=24 best_idx=20 best_idx=24 R_best=None R_best=20 R_best=24 '),
         EINVAL: (
             'vol_dtype=-1 vol_dtype=2 math_mode=-1 math_mode=3 B=-1 B=0 N=-1 N=0 N=1 N=3 N=2147483648 k=-1 k=0 '
-            'k=33 m=0 m=536870912 vol_src=None vol_src=20 vol_src=24 vol_tgt=None vol_tgt=20 vol_tgt=24 R=None '
+            'k=33 m=0 m=536870912 max_angle_deg=-1.0 max_angle_deg=181.0 max_angle_deg=nan vol_src=None '
+            'vol_src=20 vol_src=24 vol_tgt=None vol_tgt=20 vol_tgt=24 R=None '
             'R=20 R=24 W1=None W1=20 W1=24 W2=None W2=20 W2=24 b2=None base=None first_val=None first_idx=None '
             'first_R=None cand=None cand=20 cand=24 best_val=None best_idx=None workspace=None workspace=20 '
             'workspace=24 B=0,all=None N=0,all=None '),
