@@ -41,7 +41,7 @@ __device__ __forceinline__ void sort_row(uint32_t* a, int nmax) {
 
 // Insertion sort of one adjoint work list (offset of dX[vo], weight) by offset, which is unique per output voxel vo:
 // the deterministic backward sums every input voxel's contributions in this order, not in the order shared-memory
-// atomics handed out the places.  A rotation puts about 8 (at most ~12) entries on a voxel.
+// atomics handed out the places.  A rotation puts about 8 entries on a voxel (17 at most in 23 000 sampled rotations).
 __device__ __forceinline__ void sort_list(uint2* e, int n) {
   for (int i = 1; i < n; ++i) {
     const uint2 x = e[i];
