@@ -58,6 +58,9 @@ SIGNATURES = {
     "ahv_search_hierarchical_workspace_bytes": (_sz, [_i, _i, _i]),
     "ahv_search_hierarchical": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp,
                                      _sz, _vp]),
+    "ahv_search_modes_workspace_bytes": (_sz, [_i, _i, _i, _i]),
+    "ahv_search_modes": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, ctypes.c_float, _vp, _vp, _vp, _vp, _vp, _vp, _i,
+                              _i, _vp, _sz, _vp]),
     "ahv_topk_distinct": (_i, [_vp, _vp, _i, _i, _i64, _i, ctypes.c_float, _vp, _vp, _vp, _vp]),
     "ahv_posterior_mass_workspace_bytes": (_sz, [_i, _i64, _i]),
     "ahv_posterior_mass": (_i, [_vp, _vp, _i, _vp, _i, _i64, _i, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp, _sz, _vp]),

@@ -695,6 +695,85 @@ AHV_API int ahv_search_hierarchical(const void* vol_src, int vol_dtype, const fl
   return launch_gather_rotations(kids_R, 1, lidx, 0, B, nc, k, R_out, s);
 }
 
+// ---- coarse-to-fine search that keeps k distinct modes (extension) ------------------------------------------------
+namespace {
+constexpr int kMaxBeam = 8;
+
+// ahv_search_modes: [scoring workspace of the larger pass (its score region holds the base scores until the first level)
+//  | target features B*32*64 fp32 | base grid n0*9 fp32 | base slots B*n0 bytes | children [B,8kw] int64 | their rotations
+//  [B,8kw,9] fp32 | beams [B,k,w] int64 | the beams for the children generator [B,k,w] int64]
+struct ModesWs {
+  size_t tgt, grid, slot, kids, kids_R, par, gen, total;
+  ModesWs(int B, int base_level, int k, int w)
+      : tgt(std::max(VerifyWs(B, hopf_cells(base_level), 0).lists, VerifyWs(B, 8 * (int64_t)k * w, 0).lists)),
+        grid(tgt + align_up((size_t)B * kO * kP * sizeof(float), 256)),
+        slot(grid + align_up((size_t)hopf_cells(base_level) * 9 * sizeof(float), 256)),
+        kids(slot + align_up((size_t)B * hopf_cells(base_level), 256)),
+        kids_R(kids + align_up((size_t)B * 8 * k * w * sizeof(int64_t), 256)),
+        par(kids_R + align_up((size_t)B * 8 * k * w * 9 * sizeof(float), 256)),
+        gen(par + align_up((size_t)B * k * w * sizeof(int64_t), 256)),
+        total(gen + align_up((size_t)B * k * w * sizeof(int64_t), 256)) {}
+};
+
+bool modes_sizes_ok(int B, int base_level, int k, int beam) {
+  return B >= 1 && base_level >= 0 && base_level <= kHopfMaxBaseLevel && k_ok(k) && beam >= 1 && beam <= kMaxBeam;
+}
+}  // namespace
+
+AHV_API size_t ahv_search_modes_workspace_bytes(int B, int base_level, int k, int beam) {
+  return modes_sizes_ok(B, base_level, k, beam) ? ModesWs(B, base_level, k, beam).total : 0;
+}
+
+AHV_API int ahv_search_modes(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* W1, const float* W2,
+                             const float* b2, const float* base, int base_level, int levels, int k, int beam, float min_sep_deg,
+                             float* first_val, int64_t* first_idx, float* first_R, float* val, int64_t* idx, float* R_out, int B,
+                             int math_mode, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!modes_sizes_ok(B, base_level, k, beam) || !vol_dtype_ok(vol_dtype) || !math_mode_ok(math_mode)) return AHV_EINVAL;
+  if (levels < 0 || base_level + levels > kHopfMaxLevel) return AHV_EINVAL;
+  if (!std::isfinite(min_sep_deg) || !(min_sep_deg > 0.0f) || min_sep_deg > 180.0f) return AHV_EINVAL;
+  if (!all_set(vol_src, vol_tgt, W1, W2, b2, base, first_val, first_idx, first_R, val, idx, R_out, workspace))
+    return AHV_EINVAL;
+  if (!all_aligned16(vol_src, vol_tgt, W1, W2, first_R, R_out, workspace)) return AHV_EINVAL;
+  const ModesWs w(B, base_level, k, beam);
+  if (workspace_bytes < w.total) return AHV_EWORKSPACE;
+  int st = check_device();
+  if (st != AHV_OK) return st;
+  cudaStream_t s = (cudaStream_t)stream;
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  float* tgt = reinterpret_cast<float*>(ws + w.tgt);
+  float* grid = reinterpret_cast<float*>(ws + w.grid);
+  int64_t* kids = reinterpret_cast<int64_t*>(ws + w.kids);
+  float* kids_R = reinterpret_cast<float*>(ws + w.kids_R);
+  int64_t* par = reinterpret_cast<int64_t*>(ws + w.par);
+  int64_t* gen = reinterpret_cast<int64_t*>(ws + w.gen);
+  const float* sc = reinterpret_cast<const float*>(ws);  // score_chain's score region when it is given none
+  const int64_t n0 = hopf_cells(base_level), nc = 8 * (int64_t)k * beam;
+  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
+  if (st == AHV_OK) st = launch_so3_hopf_grid(base_level, 0, grid, n0, s);
+  // the base level (one set shared by the B pairs; local indices are grid indices) and its k distinct winners
+  if (st == AHV_OK)
+    st = score_chain(vol_src, vol_dtype, tgt, grid, 0, W1, W2, b2, base, nullptr, nullptr, nullptr, 0, 0, B, n0, math_mode, ws,
+                     s);
+  if (st == AHV_OK) st = launch_topk_distinct(sc, grid, 0, B, n0, k, min_sep_deg, first_val, first_idx, first_R, s);
+  if (st != AHV_OK) return st;
+  if (levels == 0) {
+    AHV_CUDA_OK(cudaMemcpyAsync(val, first_val, (size_t)B * k * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    AHV_CUDA_OK(cudaMemcpyAsync(idx, first_idx, (size_t)B * k * sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
+    AHV_CUDA_OK(cudaMemcpyAsync(R_out, first_R, (size_t)B * k * 9 * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    return AHV_OK;
+  }
+  st = launch_modes_beams(sc, grid, n0, first_idx, first_R, B, k, beam, min_sep_deg, ws + w.slot, par, gen, s);
+  // each level scores the children of every beam as a per-pair set [B, 8kw] and keeps each slot's top-w
+  for (int l = 0; l < levels && st == AHV_OK; ++l) {
+    st = launch_so3_hopf_children(base_level + l, gen, (int64_t)B * k * beam, kids, kids_R, s);
+    if (st == AHV_OK)
+      st = score_chain(vol_src, vol_dtype, tgt, kids_R, 1, W1, W2, b2, base, nullptr, nullptr, nullptr, 0, 0, B, nc, math_mode,
+                       ws, s);
+    if (st == AHV_OK) st = launch_modes_level(sc, kids, kids_R, B, k, beam, l == levels - 1, par, gen, val, idx, R_out, s);
+  }
+  return st;
+}
+
 // ---- top-k of distinct rotations: greedy geodesic non-maximum suppression on SO(3) (extension) ------------
 AHV_API int ahv_topk_distinct(const float* scores, const float* R, int r_per_pair, int B, int64_t N, int k,
                               float min_sep_deg, float* topk_val, int64_t* topk_idx, float* R_best, void* stream) {

@@ -237,6 +237,13 @@ int launch_gather_rotations(const float* R, int r_per_pair, const int64_t* idx, 
                             int B, int64_t N, int k, float* R_out, cudaStream_t s);
 int launch_topk_distinct(const float* scores, const float* R, int r_per_pair, int B, int64_t N, int k, float min_sep_deg,
                          float* val, int64_t* idx, float* R_best, cudaStream_t s);
+// ahv_search_modes (ahv_topk_distinct.cu): the slot of every base cell (slot [B, n0] bytes) and each slot's initial beam
+// of w cells; then per level, from the scored children [B, 8kw] of the beams, the next beams or (last) the ordered
+// modes.  par [B,k,w]: beams ascending, -1 last; gen: the same with -1 replaced by cell 0, for the children generator.
+int launch_modes_beams(const float* S0, const float* G, int64_t n0, const int64_t* first_idx, const float* first_R, int B,
+                       int k, int w, float min_sep_deg, uint8_t* slot, int64_t* par, int64_t* gen, cudaStream_t s);
+int launch_modes_level(const float* sc, const int64_t* kids, const float* kids_R, int B, int k, int w, bool last,
+                       int64_t* par, int64_t* gen, float* val, int64_t* idx, float* R_out, cudaStream_t s);
 // Screened arg-max of ahv_verify (k = 1, fp32 volumes, AHV_MATH_TC; the passes are described at
 // launch_verify_tc_screened in ahv_score_tc.cu).  Per pair a list of kScreenList hypotheses: the contenders (16-bit
 // gather score within 2 tau of the pair's screened maximum, at most kScreenCap of them, padded with the first), then

@@ -19,9 +19,10 @@
 // No workspace, no atomics, no host synchronisation: deterministic and CUDA-graph capturable.
 #include <cooperative_groups.h>
 
+#include <algorithm>
 #include <cmath>
 
-#include "ahv_common.cuh"
+#include "ahv_topk.cuh"
 
 namespace ahv {
 namespace cg = cooperative_groups;
@@ -580,6 +581,168 @@ int launch_posterior(const float* scores, const float* R, int r_per_pair, const 
     posterior_final_kernel<false><<<(unsigned)B, kFinalThreads, 0, s>>>(ws_sum, ws_max, w.chunks, k, T, log_z, mass,
                                                                         nullptr, nullptr, nullptr, nullptr);
   }
+  AHV_CUDA_OK(cudaGetLastError());
+  return AHV_OK;
+}
+
+// Coarse-to-fine search that keeps k distinct modes (ahv_search_modes; DESIGN.md §4.8.1).  With the distinct winners
+// c_j of the base level (ahv_topk_distinct) as centres, base cell n belongs to slot j when n = c_j, else to the lowest
+// slot j with t(n, c_j) >= c (the posterior mass's rule, trace_rn and trace_threshold above): slot j holds its winner and
+// the cells that winner suppressed, and c_j is the slot's largest key.  Each slot keeps a beam of w <= 8 cells of the
+// current level, ascending in grid index and padded with -1 at the end; a level scores the 8 children of every beam cell
+// as one per-pair set [B, 8kw], slot j's children being the segment [8wj, 8w(j+1)), and keeps the top-w of each
+// segment.  One CTA per pair, warp j serving slot j, keeps every selection in ahv_topk's key order.
+namespace modes {
+constexpr int kSlotThreads = 256;
+constexpr int kBeamBatch = 4;  // cells per lane whose loads a beam warp issues at once
+constexpr uint8_t kNoSlot = 0xFF;
+
+// slot[b, n] of every base cell, grid (cells / kSlotThreads, pairs)
+__global__ void __launch_bounds__(kSlotThreads)
+modes_slot_kernel(const float* __restrict__ G, int64_t n0, const int64_t* __restrict__ first_idx,
+                  const float* __restrict__ first_R, int B, int k, float c, uint8_t* __restrict__ slot) {
+  __shared__ float s_cen[kMaxK][9];
+  __shared__ int64_t s_win[kMaxK];
+  for (int b = blockIdx.y; b < B; b += gridDim.y) {
+    __syncthreads();  // the previous pair's centres are no longer read
+    for (int e = threadIdx.x; e < k * 9; e += kSlotThreads) s_cen[e / 9][e % 9] = __ldg(first_R + (size_t)b * k * 9 + e);
+    for (int j = threadIdx.x; j < k; j += kSlotThreads) s_win[j] = __ldg(first_idx + (size_t)b * k + j);
+    __syncthreads();
+    for (int64_t n = (int64_t)blockIdx.x * kSlotThreads + threadIdx.x; n < n0; n += (int64_t)gridDim.x * kSlotThreads) {
+      float a[9];
+#pragma unroll
+      for (int e = 0; e < 9; ++e) a[e] = __ldg(G + n * 9 + e);
+      int s = kNoSlot;
+      for (int j = 0; j < k; ++j) {
+        if (s_win[j] == n) {
+          s = j;
+          break;
+        }
+      }
+      if (s == kNoSlot) {
+#pragma unroll 1
+        for (int j = 0; j < k; ++j) {
+          if (distinct::trace_rn(a, s_cen[j]) >= c) {  // a NaN centre (empty slot) never passes
+            s = j;
+            break;
+          }
+        }
+      }
+      slot[(size_t)b * n0 + n] = (uint8_t)s;
+    }
+  }
+}
+
+// The w best keys of a warp's sorted list (lanes < w) as cells, written ascending with -1 last to par and, with the -1
+// replaced by cell 0 of the level (a valid rotation for the children generator), to gen.
+__device__ __forceinline__ void write_beam(u64 best, const int64_t* cells, int w, int lane, int64_t* par, int64_t* gen) {
+  int64_t v = -1;
+  if (lane < w && best != 0ull) v = cells ? cells[key_index(best)] : (int64_t)key_index(best);
+  const uint64_t ord = (uint64_t)v;  // -1 sorts after every cell
+  int pos = 0;
+  for (int i = 0; i < w; ++i) {
+    const uint64_t u = (uint64_t)__shfl_sync(0xffffffffu, v, i);
+    pos += (u < ord) || (u == ord && i < lane);
+  }
+  if (lane < w) {
+    par[pos] = v;
+    gen[pos] = v < 0 ? 0 : v;
+  }
+}
+
+// The initial beams: warp j keeps the top-w keys of slot j's cells.  Block (pair), k warps.
+__global__ void __launch_bounds__(kMaxK * 32)
+modes_beam_kernel(const float* __restrict__ S0, const uint8_t* __restrict__ slot, int64_t n0, int k, int w,
+                  int64_t* __restrict__ par, int64_t* __restrict__ gen) {
+  const int b = blockIdx.x, j = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const float* row = S0 + (size_t)b * n0;
+  const uint8_t* sl = slot + (size_t)b * n0;
+  u64 best = 0ull;
+  for (int64_t i = 0; i < n0; i += 32 * kBeamBatch) {  // a batch's loads in flight together: the scan is latency-bound
+    u64 cand[kBeamBatch];
+#pragma unroll
+    for (int u = 0; u < kBeamBatch; ++u) {
+      const int64_t n = i + u * 32 + lane;
+      cand[u] = n < n0 && __ldg(sl + n) == j ? make_key(__ldg(row + n), (uint32_t)n) : 0ull;
+    }
+#pragma unroll
+    for (int u = 0; u < kBeamBatch; ++u) best = warp_offer(best, cand[u], lane);
+  }
+  const size_t at = ((size_t)b * k + j) * w;
+  write_beam(best, nullptr, w, lane, par + at, gen + at);
+}
+
+// One level: warp j keeps the top-w of segment j of the pair's scored children (a -1 parent's 8 children never
+// qualify).  Not the last level: the beams of the next.  The last: each slot's best, then warp 0 orders the k modes by
+// key (score descending, ties to the lower grid index; empty modes last, in slot order) into val, idx and R_out.
+__global__ void __launch_bounds__(kMaxK * 32)
+modes_level_kernel(const float* __restrict__ sc, const int64_t* __restrict__ kids, const float* __restrict__ kids_R, int k,
+                   int w, bool last, int64_t* __restrict__ par, int64_t* __restrict__ gen, float* __restrict__ val,
+                   int64_t* __restrict__ idx, float* __restrict__ R_out) {
+  __shared__ u64 s_key[kMaxK];
+  __shared__ int64_t s_cell[kMaxK];
+  const int b = blockIdx.x, j = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int nc = 8 * w;
+  const size_t seg = ((size_t)b * k + j) * nc, at = ((size_t)b * k + j) * w;
+  u64 best = 0ull;
+#pragma unroll
+  for (int h = 0; h < 64; h += 32) {
+    const int t = h + lane;
+    const bool real = t < nc && par[at + (t >> 3)] >= 0;
+    best = warp_offer(best, real ? make_key(__ldg(sc + seg + t), (uint32_t)t) : 0ull, lane);
+  }
+  if (!last) {  // a warp overwrites only the parents it has read
+    write_beam(best, kids + seg, w, lane, par + at, gen + at);
+    return;
+  }
+  if (lane == 0) {
+    s_key[j] = best;
+    s_cell[j] = best != 0ull ? kids[seg + key_index(best)] : -1;
+  }
+  __syncthreads();
+  if (j != 0) return;
+  const u64 key = lane < k ? s_key[lane] : 0ull;
+  const uint32_t hi = (uint32_t)(key >> 32);
+  const uint64_t tie = key != 0ull ? (uint64_t)s_cell[lane] : (uint64_t)lane;  // empty: hi == 0, in slot order
+  int pos = 0;
+  for (int i = 0; i < k; ++i) {
+    const uint32_t hi_i = __shfl_sync(0xffffffffu, hi, i);
+    const uint64_t tie_i = __shfl_sync(0xffffffffu, tie, i);
+    pos += hi_i > hi || (hi_i == hi && tie_i < tie);
+  }
+  if (lane >= k) return;
+  const size_t o = (size_t)b * k + pos;
+  idx[o] = s_cell[lane];
+  if (key == 0ull) {
+    val[o] = -INFINITY;
+#pragma unroll
+    for (int e = 0; e < 9; ++e) R_out[o * 9 + e] = nanf("");
+    return;
+  }
+  val[o] = key_score(key);
+  const float* src = kids_R + (((size_t)b * k + lane) * nc + key_index(key)) * 9;
+#pragma unroll
+  for (int e = 0; e < 9; ++e) R_out[o * 9 + e] = src[e];
+}
+}  // namespace modes
+
+int launch_modes_beams(const float* S0, const float* G, int64_t n0, const int64_t* first_idx, const float* first_R, int B,
+                       int k, int w, float min_sep_deg, uint8_t* slot, int64_t* par, int64_t* gen, cudaStream_t s) {
+  using namespace modes;
+  if (B == 0) return AHV_OK;
+  const unsigned gx = (unsigned)std::min<int64_t>((n0 + kSlotThreads - 1) / kSlotThreads, 1 << 16);
+  modes_slot_kernel<<<dim3(gx, (unsigned)(B < 65535 ? B : 65535)), kSlotThreads, 0, s>>>(
+      G, n0, first_idx, first_R, B, k, distinct::trace_threshold(min_sep_deg), slot);
+  AHV_CUDA_OK(cudaGetLastError());
+  modes_beam_kernel<<<(unsigned)B, 32 * k, 0, s>>>(S0, slot, n0, k, w, par, gen);
+  AHV_CUDA_OK(cudaGetLastError());
+  return AHV_OK;
+}
+
+int launch_modes_level(const float* sc, const int64_t* kids, const float* kids_R, int B, int k, int w, bool last,
+                       int64_t* par, int64_t* gen, float* val, int64_t* idx, float* R_out, cudaStream_t s) {
+  if (B == 0) return AHV_OK;
+  modes::modes_level_kernel<<<(unsigned)B, 32 * k, 0, s>>>(sc, kids, kids_R, k, w, last, par, gen, val, idx, R_out);
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }

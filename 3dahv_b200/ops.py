@@ -183,6 +183,43 @@ def search_hierarchical(vol_src, vol_tgt, W1, W2, b2, base_level: int = 2, level
     return fv, fi, fR, v, i, R, workspace
 
 
+def search_modes_workspace_bytes(B: int, base_level: int, k: int, beam: int) -> int:
+    """Bytes of scratch `search_modes` needs (0 for invalid sizes); it holds the base grid, 36 B per cell, and one slot
+    byte per cell and pair."""
+    return int(_lib.lib().ahv_search_modes_workspace_bytes(B, base_level, k, beam))
+
+
+def search_modes(vol_src, vol_tgt, W1, W2, b2, base_level: int = 2, levels: int = 4, k: int = 8, beam: int = 4,
+                 min_sep_deg: float = 30.0, math: int = MATH_TC, workspace: torch.Tensor | None = None, out=None):
+    """ahv_search_modes: coarse-to-fine search that keeps k distinct modes, in one C call.  The whole base level is scored
+    and its k distinct winners taken (`topk_distinct(min_sep_deg)`); every base cell joins the lowest slot whose winner
+    lies within min_sep_deg of it (the winner's own slot for the winner), and each slot descends `levels` levels with a
+    beam of its own `beam` best cells, their children scored per pair.  No torch ops, no host synchronisation,
+    CUDA-graph capturable (pass `out` = the tuple a previous call returned to reuse its buffers).  Returns (first_val
+    [B,k], first_idx [B,k], first_R [B,k,3,3] - the base level's distinct winners, indices of level base_level - val
+    [B,k], idx [B,k], R [B,k,3,3] - each mode's best cell at level base_level + levels, ordered by score; slot 0 is the
+    answer - workspace).  Empty modes (fewer than k distinct winners) are -inf / -1 / NaN, last."""
+    vs, vdt, vt, B = _vols(vol_src, vol_tgt)
+    if not (1 <= k <= 32 and 1 <= beam <= 8 and 0 <= base_level <= HOPF_MAX_BASE_LEVEL and levels >= 0
+            and base_level + levels <= HOPF_MAX_LEVEL):
+        raise ValueError("1 <= k <= 32, 1 <= beam <= 8, 0 <= base_level <= 6, levels >= 0 and base_level + levels <= 16 "
+                         "expected")
+    if not 0 < min_sep_deg <= 180:
+        raise ValueError("0 < min_sep_deg <= 180 expected")
+    W1, W2, b2 = _head(W1, W2, b2)
+    dev = vs.device
+    if out is None:
+        f = dict(device=dev, dtype=torch.float32)
+        out = (torch.empty(B, k, **f), torch.empty(B, k, device=dev, dtype=torch.int64), torch.empty(B, k, 3, 3, **f),
+               torch.empty(B, k, **f), torch.empty(B, k, device=dev, dtype=torch.int64), torch.empty(B, k, 3, 3, **f))
+    fv, fi, fR, v, i, R = out[:6]
+    workspace, ws_bytes = _workspace(workspace, search_modes_workspace_bytes(B, base_level, k, beam), dev)
+    _call("ahv_search_modes", dev, vs.data_ptr(), vdt, vt.data_ptr(), W1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
+          base_coords(dev).data_ptr(), int(base_level), int(levels), int(k), int(beam), float(min_sep_deg), fv.data_ptr(),
+          fi.data_ptr(), fR.data_ptr(), v.data_ptr(), i.data_ptr(), R.data_ptr(), B, int(math), workspace.data_ptr(), ws_bytes)
+    return fv, fi, fR, v, i, R, workspace
+
+
 def perturb_rotations(R_center: torch.Tensor, m: int, max_angle_deg: float, seed: int = 0) -> torch.Tensor:
     """ahv_so3_perturb: [...,3,3] centres -> [...,m,3,3] rotations within `max_angle_deg` of them (index 0 = the
     centre itself)."""

@@ -278,7 +278,8 @@ class HypothesisVerifier:
 
 
     @torch.no_grad()
-    def search(self, vol_src, vol_tgt, base_level: int = 2, levels: int = 4, k: int = 32):
+    def search(self, vol_src, vol_tgt, base_level: int = 2, levels: int = 4, k: int = 32, min_sep_deg: float = 0.0,
+               beam: int = 4):
         """Coarse-to-fine rotation search on the nested Hopf x HEALPix grid (`so3.hopf_grid`) in one C call
         (`ahv_search_hierarchical`): score all 72 * 8^base_level cells of the base level with this verifier's math mode,
         keep the top-k, then `levels` times score the 8 children of each kept cell and keep the top-k of those.  It
@@ -289,9 +290,26 @@ class HypothesisVerifier:
         more than that grid; k = 32 reaches the dense grid's top-1 score on 96.5 % of 256 random pairs against 89.5 % for
         k = 8, for 6-15 % more time; four levels end on 0.46-deg cells, below the 50 000-point grid's 3.3 deg.  A coarse base
         level can miss the right basin: on near-symmetric volumes only base_level=3 with k=32 found every pair's mode.
+        min_sep_deg > 0 keeps k distinct modes instead (`ops.search_modes`, `ahv_search_modes`): the base level's k winners
+        pairwise more than min_sep_deg apart, each descended with a beam of its own `beam` best cells, so a second peak
+        that scores a little lower is not dropped at the coarse level.  `first` then holds the distinct base winners and
+        `final` the k modes ordered by score.  On near-symmetric volumes (profiles/r18_search_modes.jsonl, B200) the modes
+        at (2, 4, k=8, beam=4, 30 deg) held every pair's true basin, but the top-1 was often the mirrored peak: `ascend`
+        from every mode and take the best score (0.035 deg at most there).  Empty modes (fewer than k distinct winners) carry score -inf, index -1
+        and NaN rotations: filter them (final.topk_idx >= 0) before passing final.R_best to `ascend`.  `beam` applies to
+        min_sep_deg > 0 only.
         Returns (R_best [B,3,3], score [B], first: VerifyResult of the base level's top-k, final: VerifyResult of the
         finest level's top-k); the VerifyResults carry grid indices of their level and no scores."""
+        if not min_sep_deg >= 0:
+            raise ValueError("min_sep_deg must be >= 0")
         W1, W2, b2 = self._weights_on(vol_src.device)
+        if min_sep_deg > 0:
+            fv, fi, fR, v, i, R, self._ws_search_modes = ops.search_modes(
+                _src_volume(vol_src), vol_tgt.float(), W1, W2, b2, base_level=base_level, levels=levels, k=k, beam=beam,
+                min_sep_deg=min_sep_deg, math=self.math, workspace=getattr(self, "_ws_search_modes", None))
+            return R[:, 0], v[:, 0], VerifyResult(None, fv, fi, fR), VerifyResult(None, v, i, R)
+        if beam != 4:
+            raise ValueError("beam applies to min_sep_deg > 0 only")
         fv, fi, fR, v, i, R, self._ws_search = ops.search_hierarchical(
             _src_volume(vol_src), vol_tgt.float(), W1, W2, b2, base_level=base_level, levels=levels, k=k, math=self.math,
             workspace=getattr(self, "_ws_search", None))

@@ -352,6 +352,36 @@ AHV_API int ahv_search_hierarchical(const void* vol_src, int vol_dtype, const fl
                                     int64_t* first_idx, float* first_R, float* val, int64_t* idx, float* R_out, int B,
                                     int math_mode, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Coarse-to-fine search that keeps k DISTINCT modes (extension), one call.  ahv_search_hierarchical keeps the global
+ * top-k of every level, whose cells can crowd around one peak; this search descends each mode with a beam of its own:
+ *   target features once; the whole base_level grid (72*8^base_level cells) generated into the workspace and scored
+ *   with ahv_score(k = 0, math_mode), giving S0 [B,n0];
+ *   modes: first_val [B,k], first_idx [B,k], first_R [B,k,3,3] = ahv_topk_distinct(S0, grid, k, min_sep_deg) bit for bit
+ *   (empty slots -inf / -1 / NaN);
+ *   slots: base cell n goes to slot j when n = first_idx[j], else to the lowest non-empty slot j with
+ *   t(n, first_R[j]) >= c (t and c are ahv_topk_distinct's, the rule of ahv_posterior_mass), so slot j holds its winner
+ *   and the cells that winner suppressed; cells of no slot are dropped;
+ *   beams: slot j's beam is the top-`beam` cells of the slot in ahv_topk's key order (the winner first), kept in
+ *   ascending grid index and padded with -1 at the end;
+ *   each of `levels` levels: the 8 children of every beam cell form a per-pair set [B, 8*k*beam], slot-major (slot j's
+ *   children are the segment [8*beam*j, 8*beam*(j+1)), ascending in grid index), scored with ahv_score(k = 0,
+ *   math_mode); a child inherits its parent's slot, the children of a -1 pad never qualify, and slot j's next beam is
+ *   the top-`beam` of its segment (ties to the lowest grid index).
+ * val [B,k], idx [B,k] (grid indices of level base_level + levels) and R_out [B,k,3,3] (= ahv_so3_hopf_grid of that level
+ * at idx) are the best cell of each final beam, ordered by key (score descending, ties to the lower index; slot 0 is the
+ * answer), empty modes last as -inf / -1 / NaN.  The final modes are not suppressed again: two may lie close together.
+ * levels = 0 gives first_* bit for bit.  Each pair scores 72*8^base_level + levels*8*k*beam hypotheses.
+ * Rules: ahv_search_hierarchical's (0 <= base_level <= 6, base_level + levels <= 16, 1 <= k <= 32, B >= 1, every buffer
+ * required, rotation buffers, volumes, W1, W2 and the workspace 16-byte aligned), plus 1 <= beam <= 8 and a finite
+ * 0 < min_sep_deg <= 180.  Workspace: ahv_search_modes_workspace_bytes(B, base_level, k, beam) (0 for invalid sizes),
+ * which holds the base grid and one slot byte per base cell and pair.  No allocation, no host synchronisation: CUDA-graph
+ * capturable. */
+AHV_API size_t ahv_search_modes_workspace_bytes(int B, int base_level, int k, int beam);
+AHV_API int ahv_search_modes(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* W1, const float* W2,
+                             const float* b2, const float* base, int base_level, int levels, int k, int beam, float min_sep_deg,
+                             float* first_val, int64_t* first_idx, float* first_R, float* val, int64_t* idx, float* R_out, int B,
+                             int math_mode, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Top-k of distinct rotations (extension): greedy geodesic non-maximum suppression on SO(3) over the score-sorted
  * hypotheses of each pair.  With key(n) = ahv_topk's order (score descending, ties -> lowest index, NaN as ahv_topk
  * orders it), t(a,b) = trace(R_a R_b^T) in fp32 (nine individually rounded products summed left to right, no FMA) and
