@@ -30,25 +30,47 @@ int check_device() {
   return major == 10 ? AHV_OK : AHV_ENOTSUP;
 }
 
-size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+// Workspace layouts.  Each is built from the workspace's base, or from nullptr when only its size `total` is wanted, and
+// places its regions with a Carve, each 256-byte aligned.
 
-// Workspace layouts: the offset of each region (each 256-byte aligned) and the size of the whole.
-// The verification workspace: [scores B*N fp32 | top-k partials | tensor-core scratch | per-shard top-k lists].
-// ahv_score needs the bytes up to `lists` only.
+// The verification workspace: [scores B*N fp32 | top-k partials | tensor-core scratch | a shard's top-k lists [B,k]].
+// ahv_score needs the bytes before the lists, `score_bytes`.
 struct VerifyWs {
-  size_t topk, tc, lists, total;
-  VerifyWs(int B, int64_t N, int k)
-      : topk(align_up((size_t)B * (size_t)N * sizeof(float), 256)),
-        tc(topk + align_up(topk_workspace_bytes(B, N, k), 256)),
-        lists(tc + align_up(score_tc_workspace_bytes(B, N), 256)),
-        total(lists + align_up((size_t)B * (size_t)(k > 0 ? k : 1) * (sizeof(float) + sizeof(int64_t)), 256)) {}
+  float* scores;        // where score_chain scores when it is given no output
+  size_t topk_bytes;
+  unsigned char* topk;
+  ScreenLists screen;   // the screened arg-max's lists, inside the top-k partials, which it leaves unused
+  TcScratch tc;         // tc.tgt_feat: where verify_chain computes the target features
+  float* l_val;
+  int64_t* l_idx;
+  size_t score_bytes, total;
+  VerifyWs(void* ws, int B, int64_t N, int k) {
+    Carve c(ws);
+    scores = c.take<float>((size_t)B * N, 256);
+    topk_bytes = (topk_workspace_bytes(B, N, k) + 255) / 256 * 256;
+    topk = c.take<unsigned char>(topk_bytes, 256);
+    Carve in_topk(topk);
+    screen = ScreenLists(in_topk, B);
+    Carve in_tc(c.take<unsigned char>(bytes_of<TcScratch>(B), 256));
+    tc = TcScratch(in_tc, B);
+    score_bytes = c.off;
+    Carve in_lists(c.take<unsigned char>((size_t)B * (k > 0 ? k : 1) * (sizeof(float) + sizeof(int64_t)), 256));
+    l_val = in_lists.take<float>((size_t)B * k, 8);
+    l_idx = in_lists.take<int64_t>((size_t)B * k, 8);
+    total = c.off;
+  }
 };
 
 // ahv_refine: [the grid pass's verification workspace | the candidate pass's ([B, k*m], arg-max)]
 struct RefineWs {
-  size_t cand, total;
-  RefineWs(int B, int64_t N, int k, int m)
-      : cand(VerifyWs(B, N, k).total), total(cand + VerifyWs(B, (int64_t)k * m, 1).total) {}
+  unsigned char *grid, *cand;
+  size_t total;
+  RefineWs(void* ws, int B, int64_t N, int k, int m) {
+    Carve c(ws);
+    grid = c.take<unsigned char>(VerifyWs(nullptr, B, N, k).total, 256);
+    cand = c.take<unsigned char>(VerifyWs(nullptr, B, (int64_t)k * m, 1).total, 256);
+    total = c.off;
+  }
 };
 
 // ahv_refine_gradient(_distinct) (world == 1) and ahv_refine_gradient_sharded, per = ceil(N / world) hypotheses at most
@@ -56,13 +78,21 @@ struct RefineWs {
 // pass 1) | target features B*32*64 | top-k partials over [B,k]].  One GPU scores R in place and keeps the distinct
 // pass's scores in the verification workspace, so its two middle regions are empty.
 struct ShardedRefineWs {
-  size_t rs, full, tgt, top, total;
-  ShardedRefineWs(int B, int64_t N, int k, int world)
-      : rs(VerifyWs(B, (N + world - 1) / world, k).total),
-        full(rs + (world > 1 ? align_up((size_t)B * (size_t)((N + world - 1) / world) * 9 * sizeof(float), 256) : 0)),
-        tgt(full + (world > 1 ? align_up((size_t)B * (size_t)N * sizeof(float), 256) : 0)),
-        top(tgt + align_up((size_t)B * kO * kP * sizeof(float), 256)),
-        total(top + align_up(topk_workspace_bytes(B, k, 1), 256)) {}
+  unsigned char* verify;
+  float *rs, *full, *tgt;
+  unsigned char* top;
+  size_t top_bytes, total;
+  ShardedRefineWs(void* ws, int B, int64_t N, int k, int world) {
+    const int64_t per = (N + world - 1) / world;
+    Carve c(ws);
+    verify = c.take<unsigned char>(VerifyWs(nullptr, B, per, k).total, 256);
+    rs = c.take<float>(world > 1 ? (size_t)B * (size_t)per * 9 : 0, 256);
+    full = c.take<float>(world > 1 ? (size_t)B * (size_t)N : 0, 256);
+    tgt = c.take<float>((size_t)B * kO * kP, 256);
+    top_bytes = (topk_workspace_bytes(B, k, 1) + 255) / 256 * 256;
+    top = c.take<unsigned char>(top_bytes, 256);
+    total = c.off;
+  }
 };
 
 // The screened arg-max (launch_verify_tc_screened, ahv_score_tc.cu) serves ahv_verify and ahv_verify_sharded for fp32
@@ -73,7 +103,7 @@ struct ShardedRefineWs {
 constexpr int64_t kScreenMinItems = 1 << 18;
 bool screened(const VerifyWs& w, int vol_dtype, int math_mode, const float* scores, int k, int B, int64_t N) {
   return vol_dtype == AHV_VOL_F32 && math_mode == AHV_MATH_TC && k == 1 && !scores && (int64_t)B * N >= kScreenMinItems &&
-         N * sizeof(float) >= kScreenList * 10 * sizeof(float) && w.tc - w.topk >= ScreenLists::bytes(B);
+         N * sizeof(float) >= kScreenList * 10 * sizeof(float) && w.topk_bytes >= bytes_of<ScreenLists>(B);
 }
 
 // dist.shard_bounds: rank's contiguous share [lo, hi) of n items
@@ -88,141 +118,109 @@ void shard_bounds(int64_t n, int rank, int world, int64_t* lo, int64_t* hi) {
 // another (the host-buffer entries aside).  `pa` == nullptr or a group of one is one GPU.
 
 // ahv_score: the scores (into `scores`, else the workspace's score region) and, for k > 0, their top-k
-int score_chain(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R, int r_per_pair, const float* W1,
-                const float* W2, const float* b2, const float* base, float* scores, float* topk_val, int64_t* topk_idx, int k,
-                int64_t idx_offset, int B, int64_t N, int math_mode, unsigned char* ws, cudaStream_t s) {
-  const VerifyWs w(B, N, k);
-  float* sc = scores ? scores : reinterpret_cast<float*>(ws);
-  int st;
-  if (math_mode == AHV_MATH_FP32)
-    st = launch_score_fp32(vol_src, vol_dtype, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, sc, B, N, s);
-  else
-    st = launch_score_tc(vol_src, vol_dtype, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, sc, B, N, ws + w.tc,
-                         w.lists - w.tc, s, math_mode == AHV_MATH_TC_F16GATHER);
-  if (st != AHV_OK) return st;
-  if (k > 0) st = launch_topk(sc, B, N, k, idx_offset, topk_val, topk_idx, ws + w.topk, w.tc - w.topk, s);
-  return st;
+int score_chain(const Scored& p, const float* tgt_feat, float* scores, float* topk_val, int64_t* topk_idx, int k,
+                int64_t idx_offset, int math_mode, void* ws, cudaStream_t s) {
+  const VerifyWs w(ws, p.B, p.N, k);
+  float* sc = scores ? scores : w.scores;
+  const int st = math_mode == AHV_MATH_FP32 ? launch_score_fp32(p, tgt_feat, sc, s)
+                                            : launch_score_tc(p, tgt_feat, sc, w.tc, s, math_mode == AHV_MATH_TC_F16GATHER);
+  if (st != AHV_OK || k == 0) return st;
+  return launch_topk(sc, p.B, p.N, k, idx_offset, topk_val, topk_idx, w.topk, w.topk_bytes, s);
 }
 
 // ahv_verify (B*N > 0) and a shard's step of ahv_verify_sharded (N == 0: an empty shard, which still joins the exchange).
-// The fused launchers get the caller's scratch from the tensor-core region on: its end on one GPU, `lists` on a shard,
-// whose per-shard lists follow.  A shard returns the whole set's selection only, so it passes no scores.
-int verify_chain(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair, const float* W1,
-                 const float* W2, const float* b2, const float* base, float* scores, float* topk_val, int64_t* topk_idx,
-                 float* R_best, int k, int64_t idx_offset, int B, int64_t N, int math_mode, void* workspace,
-                 size_t workspace_bytes, cudaStream_t s, const peer::Args* pa) {
+// A shard returns the whole set's selection only, so it passes no scores.
+int verify_chain(const Scored& p, const float* vol_tgt, float* scores, float* topk_val, int64_t* topk_idx, float* R_best,
+                 int k, int64_t idx_offset, int math_mode, void* ws, cudaStream_t s, const peer::Args* pa) {
   if (pa && pa->world == 1) pa = nullptr;
-  const VerifyWs w(B, N, k);
-  unsigned char* ws = static_cast<unsigned char*>(workspace);
-  const size_t tc_bytes = pa ? w.lists - w.tc : workspace_bytes - w.tc;  // packed weights, target features, scales, keys
-  if (N > 0 && screened(w, vol_dtype, math_mode, scores, k, B, N))  // a shard's last pass exchanges and merges the winners
-    return launch_verify_tc_screened(static_cast<const float*>(vol_src), vol_tgt, R, r_per_pair != 0, W1, W2, b2, base,
-                                     topk_val, topk_idx, R_best, idx_offset, B, N, ws + w.tc, tc_bytes,
-                                     reinterpret_cast<float*>(ws), ws + w.topk, s, pa);
+  const int B = p.B;
+  const int64_t N = p.N;
+  const VerifyWs w(ws, B, N, k);
+  if (N > 0 && screened(w, p.vol_dtype, math_mode, scores, k, B, N))  // a shard's last pass exchanges and merges the winners
+    return launch_verify_tc_screened(p, vol_tgt, topk_val, topk_idx, R_best, idx_offset, w.tc, w.scores, w.screen, s, pa);
   // three launches, nothing but 40 B per hypothesis touches HBM; a shard's scoring kernel exchanges and merges itself
   if (N > 0 && k == 1 && math_mode != AHV_MATH_FP32)
-    return launch_verify_tc_argmax(vol_src, vol_dtype, vol_tgt, R, r_per_pair != 0, W1, W2, b2, base, scores, topk_val,
-                                   topk_idx, R_best, idx_offset, B, N, ws + w.tc, tc_bytes, s,
+    return launch_verify_tc_argmax(p, vol_tgt, scores, topk_val, topk_idx, R_best, idx_offset, w.tc, s,
                                    math_mode == AHV_MATH_TC_F16GATHER, pa);
-  float* tgt = scratch_tgt_feat(ws + w.tc, B);
+  float* tgt = w.tc.tgt_feat;
   int st;
   if (!pa) {  // target features, scores and top-k, winner gather
-    st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
+    st = launch_forward_3d2d(vol_tgt, p.W1, p.W2, p.b2, tgt, B, s);
     if (st != AHV_OK) return st;
-    st = score_chain(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, scores, topk_val, topk_idx, k, idx_offset, B,
-                     N, math_mode, ws, s);
+    st = score_chain(p, tgt, scores, topk_val, topk_idx, k, idx_offset, math_mode, ws, s);
     if (st != AHV_OK || !R_best) return st;
-    return launch_gather_rotations(R, r_per_pair != 0, topk_idx, idx_offset, B, N, k, R_best, s);
+    return launch_gather_rotations(p.R, p.r_per_pair, topk_idx, idx_offset, B, N, k, R_best, s);
   }
-  // a shard with k > 1 (or empty, or fp32 FFMA arithmetic): its local top-k, then the exchange kernel
-  float* l_val = reinterpret_cast<float*>(ws + w.lists);
-  int64_t* l_idx = reinterpret_cast<int64_t*>(ws + w.lists + align_up((size_t)B * k * sizeof(float), 8));
-  const int kl = N < k ? (int)N : k;
-  if (kl < k) {  // pad with (-inf, -1), which the merge ignores
-    AHV_CUDA_OK(cudaMemsetAsync(l_val, 0xff, (size_t)B * k * sizeof(float), s));
-    AHV_CUDA_OK(cudaMemsetAsync(l_idx, 0xff, (size_t)B * k * sizeof(int64_t), s));
-  }
-  if (N > 0) {
-    st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
+  // a shard with k > 1 (or empty, or fp32 FFMA arithmetic): its local top-k, then the exchange kernel.  The top-k of a
+  // shard with fewer than k hypotheses ends in (-inf, -1), which the exchange ignores; an empty shard's list is all that.
+  if (N == 0) {
+    AHV_CUDA_OK(cudaMemsetAsync(w.l_val, 0xff, (size_t)B * k * sizeof(float), s));
+    AHV_CUDA_OK(cudaMemsetAsync(w.l_idx, 0xff, (size_t)B * k * sizeof(int64_t), s));
+  } else {
+    st = launch_forward_3d2d(vol_tgt, p.W1, p.W2, p.b2, tgt, B, s);
     if (st != AHV_OK) return st;
-    if (kl == k) {
-      st = score_chain(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, nullptr, l_val, l_idx, k, idx_offset, B, N,
-                       math_mode, ws, s);
-    } else {  // fewer hypotheses than k on this shard: compact [B,kl] lists (in the output buffers, which the
-              // exchange overwrites afterwards), then spread into the padded [B,k]
-      st = score_chain(vol_src, vol_dtype, tgt, R, r_per_pair, W1, W2, b2, base, nullptr, topk_val, topk_idx, kl, idx_offset,
-                       B, N, math_mode, ws, s);
-      if (st != AHV_OK) return st;
-      AHV_CUDA_OK(cudaMemcpy2DAsync(l_val, (size_t)k * sizeof(float), topk_val, (size_t)kl * sizeof(float),
-                                    (size_t)kl * sizeof(float), B, cudaMemcpyDeviceToDevice, s));
-      AHV_CUDA_OK(cudaMemcpy2DAsync(l_idx, (size_t)k * sizeof(int64_t), topk_idx, (size_t)kl * sizeof(int64_t),
-                                    (size_t)kl * sizeof(int64_t), B, cudaMemcpyDeviceToDevice, s));
-    }
+    st = score_chain(p, tgt, nullptr, w.l_val, w.l_idx, k, idx_offset, math_mode, ws, s);
     if (st != AHV_OK) return st;
   }
-  return launch_topk_exchange(l_val, l_idx, R, r_per_pair != 0, idx_offset, N, B, k, topk_val, topk_idx, R_best, *pa, s);
+  return launch_topk_exchange(w.l_val, w.l_idx, p.R, p.r_per_pair, idx_offset, N, B, k, topk_val, topk_idx, R_best, *pa, s);
 }
 
 // ahv_refine_gradient(_distinct) and ahv_refine_gradient_sharded: the first pass (top-k, or with min_sep_deg > 0 the
 // distinct top-k of every score), target features, gradient ascent of each winner, per-pair arg-max.  A rank of a group
 // scores its shard_bounds slice of R, exchanges the first pass, ascends its share of the B*k slots and gathers every
 // ascended slot; every rank then holds the whole-set result.
-int refine_gradient_chain(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
-                          const float* W1, const float* W2, const float* b2, const float* base, int k, int steps,
-                          float step_deg, float min_sep_deg, float* first_val, int64_t* first_idx, float* first_R,
-                          float* R_all, float* score_all, float* best_val, int64_t* best_idx, float* R_best, int B, int64_t N,
-                          int math_mode, void* workspace, cudaStream_t s, const peer::Args* pa, int64_t peer_max_hyps) {
+int refine_gradient_chain(const Scored& p, const float* vol_tgt, int k, int steps, float step_deg, float min_sep_deg,
+                          float* first_val, int64_t* first_idx, float* first_R, float* R_all, float* score_all,
+                          float* best_val, int64_t* best_idx, float* R_best, int math_mode, void* ws, cudaStream_t s,
+                          const peer::Args* pa, int64_t peer_max_hyps) {
   if (pa && pa->world == 1) pa = nullptr;
-  const ShardedRefineWs w(B, N, k, pa ? pa->world : 1);
-  unsigned char* ws = static_cast<unsigned char*>(workspace);
-  float* tgt = reinterpret_cast<float*>(ws + w.tgt);
+  const int B = p.B;
+  const int64_t N = p.N;
+  const ShardedRefineWs w(ws, B, N, k, pa ? pa->world : 1);
   const bool distinct = min_sep_deg > 0.0f;
   int64_t lo = 0, hi = N;
   if (pa) shard_bounds(N, pa->rank, pa->world, &lo, &hi);
   const int64_t n = hi - lo;
-  const float* rs = pa ? reinterpret_cast<float*>(ws + w.rs) : R;
+  const Scored slice = p.with_R(pa ? w.rs : p.R, p.r_per_pair, n);
   if (pa && n > 0)  // this rank's rotations, 16-byte aligned for the scorers (a shared set: one row)
-    AHV_CUDA_OK(cudaMemcpy2DAsync(ws + w.rs, (size_t)n * 9 * sizeof(float), R + (size_t)lo * 9, (size_t)N * 9 * sizeof(float),
-                                  (size_t)n * 9 * sizeof(float), r_per_pair ? B : 1, cudaMemcpyDeviceToDevice, s));
+    AHV_CUDA_OK(cudaMemcpy2DAsync(w.rs, (size_t)n * 9 * sizeof(float), p.R + (size_t)lo * 9, (size_t)N * 9 * sizeof(float),
+                                  (size_t)n * 9 * sizeof(float), p.r_per_pair ? B : 1, cudaMemcpyDeviceToDevice, s));
   int st;
   if (!distinct) {
     // pass 1: the top-k and their rotations (a shard's, exchanged and merged into the whole set's)
-    st = verify_chain(vol_src, vol_dtype, vol_tgt, rs, r_per_pair, W1, W2, b2, base, nullptr, first_val, first_idx, first_R, k,
-                      lo, B, n, math_mode, ws, w.rs, s, pa);
+    st = verify_chain(slice, vol_tgt, nullptr, first_val, first_idx, first_R, k, lo, math_mode, w.verify, s, pa);
     if (st != AHV_OK) return st;
   }
   // the ascent scores in fp32 against fp32 target features (bit-equal to ahv_forward_3d2d), whatever math_mode is
-  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
+  st = launch_forward_3d2d(vol_tgt, p.W1, p.W2, p.b2, w.tgt, B, s);
   if (st != AHV_OK) return st;
   if (distinct) {
     // pass 1: every score of the set (the fused k = 1 arg-max writes none), a shard's all-gathered into the whole [B,N]
     // on every rank, then the k distinct winners: the SAME greedy selection over the whole set on every rank (per-shard
     // NMS lists do not merge into the global one)
-    const float* sc = reinterpret_cast<const float*>(ws);
+    const float* sc = VerifyWs(w.verify, B, n, 0).scores;
     if (n > 0) {
-      st = score_chain(vol_src, vol_dtype, tgt, rs, r_per_pair, W1, W2, b2, base, nullptr, nullptr, nullptr, 0, 0, B, n,
-                       math_mode, ws, s);
+      st = score_chain(slice, w.tgt, nullptr, nullptr, nullptr, 0, 0, math_mode, w.verify, s);
       if (st != AHV_OK) return st;
     }
     if (pa) {
-      float* full = reinterpret_cast<float*>(ws + w.full);
-      st = launch_scores_exchange(sc, B, N, full, *pa, peer_max_hyps, s);
+      st = launch_scores_exchange(sc, B, N, w.full, *pa, peer_max_hyps, s);
       if (st != AHV_OK) return st;
-      sc = full;
+      sc = w.full;
     }
-    st = launch_topk_distinct(sc, R, r_per_pair != 0, B, N, k, min_sep_deg, first_val, first_idx, first_R, s);
+    st = launch_topk_distinct(sc, p.R, p.r_per_pair, B, N, k, min_sep_deg, first_val, first_idx, first_R, s);
     if (st != AHV_OK) return st;
   }
   // empty slots (fewer than k distinct winners) are not ascended: R_all NaN, score_all -inf.  One GPU ascends every
   // slot (item_hi < 0), a rank its share, after which every ascended slot goes to every rank.
   int64_t ilo = 0, ihi = -1;
   if (pa) shard_bounds((int64_t)B * k, pa->rank, pa->world, &ilo, &ihi);
-  st = launch_gradient_ascent(vol_src, vol_dtype, tgt, first_R, W1, W2, b2, base, steps, step_deg, R_all, score_all, B, k, s,
+  st = launch_gradient_ascent(p.with_R(first_R, true, k), w.tgt, steps, step_deg, R_all, score_all, s,
                               distinct ? first_idx : nullptr, ilo, ihi);
   if (st == AHV_OK && pa) st = launch_slot_gather(R_all, score_all, ilo, ihi, B, k, *pa, s);
   if (st != AHV_OK) return st;
   // per-pair arg-max over the k ascended candidates (on every rank)
-  st = launch_topk(score_all, B, k, 1, 0, best_val, best_idx, ws + w.top, w.total - w.top, s);
+  st = launch_topk(score_all, B, k, 1, 0, best_val, best_idx, w.top, w.top_bytes, s);
   if (st != AHV_OK || !R_best) return st;
   return launch_gather_rotations(R_all, 1, best_idx, 0, B, k, 1, R_best, s);
 }
@@ -317,8 +315,8 @@ AHV_API int ahv_score_backward(const float* vol_src, const float* tgt_feat, cons
     return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
-  return launch_score_bwd(vol_src, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, grad_scores, grad_vol, grad_tgt,
-                          grad_W1, grad_W2, grad_b2, B, N, (cudaStream_t)stream);
+  const Scored p{vol_src, AHV_VOL_F32, W1, W2, b2, base, R, r_per_pair != 0, B, N};
+  return launch_score_bwd(p, tgt_feat, grad_scores, grad_vol, grad_tgt, grad_W1, grad_W2, grad_b2, (cudaStream_t)stream);
 }
 
 AHV_API int ahv_rotate_volume_grad_R(const float* vol, int vol_per_rotation, const float* R, const float* base,
@@ -340,13 +338,14 @@ AHV_API int ahv_score_backward_ex(const float* vol_src, const float* tgt_feat, c
   if ((int64_t)B * N > 0 && !all_set(vol_src, tgt_feat, R, W1, W2, b2, base, grad_scores)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
-  return launch_score_bwd(vol_src, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, grad_scores, grad_vol, grad_tgt,
-                          grad_W1, grad_W2, grad_b2, B, N, (cudaStream_t)stream, h1_saved, pair_inv_scale, grad_R);
+  const Scored p{vol_src, AHV_VOL_F32, W1, W2, b2, base, R, r_per_pair != 0, B, N};
+  return launch_score_bwd(p, tgt_feat, grad_scores, grad_vol, grad_tgt, grad_W1, grad_W2, grad_b2, (cudaStream_t)stream,
+                          h1_saved, pair_inv_scale, grad_R);
 }
 
 AHV_API size_t ahv_score_backward_det_workspace_bytes(int B, int64_t N, int r_per_pair, int want_grad_R) {
   if (B < 0 || !n_ok(N)) return 0;
-  return DetBwdWs(B, N, want_grad_R && !r_per_pair).total * sizeof(float);
+  return bytes_of<DetBwdWs>(B, N, want_grad_R && !r_per_pair);
 }
 
 AHV_API int ahv_score_backward_det(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
@@ -362,13 +361,14 @@ AHV_API int ahv_score_backward_det(const float* vol_src, const float* tgt_feat, 
   if (!h1_saved != !pair_inv_scale) return AHV_EINVAL;
   if ((int64_t)B * N > 0 && !all_set(vol_src, tgt_feat, R, W1, W2, b2, base, grad_scores)) return AHV_EINVAL;
   if (!all_aligned16(vol_src, tgt_feat, R, W1, W2, h1_saved, workspace)) return AHV_EINVAL;
-  const DetBwdWs w(B, N, grad_R && !r_per_pair);
-  if ((int64_t)B * N > 0 && (!workspace || workspace_bytes < w.total * sizeof(float))) return AHV_EWORKSPACE;
+  Carve c(workspace);
+  const DetBwdWs w(c, B, N, grad_R && !r_per_pair);
+  if ((int64_t)B * N > 0 && (!workspace || workspace_bytes < c.off)) return AHV_EWORKSPACE;
   int st = check_device();
   if (st != AHV_OK) return st;
-  return launch_score_bwd_det(vol_src, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, grad_scores, h1_saved,
-                              pair_inv_scale, grad_vol, grad_tgt, grad_W1, grad_W2, grad_b2, grad_R, B, N,
-                              h1_saved && math_mode == AHV_MATH_TC, static_cast<float*>(workspace), (cudaStream_t)stream);
+  const Scored p{vol_src, AHV_VOL_F32, W1, W2, b2, base, R, r_per_pair != 0, B, N};
+  return launch_score_bwd_det(p, tgt_feat, grad_scores, h1_saved, pair_inv_scale, grad_vol, grad_tgt, grad_W1, grad_W2,
+                              grad_b2, grad_R, h1_saved && math_mode == AHV_MATH_TC, w, (cudaStream_t)stream);
 }
 
 AHV_API int ahv_infonce(const float* scores, const float* R, int r_per_pair, const float* gt_R, float acc_thr_deg,
@@ -399,8 +399,11 @@ AHV_API int ahv_score_train(const float* vol_src, const float* tgt_feat, const f
   if (!all_aligned16(vol_src, tgt_feat, R, W1, W2, h1_saved, workspace)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
-  return launch_score_tc_train(vol_src, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, scores, h1_saved, pair_inv_scale, B, N,
-                               workspace, workspace_bytes, (cudaStream_t)stream);
+  if ((int64_t)B * N == 0) return AHV_OK;
+  if (workspace_bytes < bytes_of<TcScratch>(B)) return AHV_EWORKSPACE;
+  Carve c(workspace);
+  const Scored p{vol_src, AHV_VOL_F32, W1, W2, b2, base, R, r_per_pair != 0, B, N};
+  return launch_score_tc_train(p, tgt_feat, scores, h1_saved, pair_inv_scale, TcScratch(c, B), (cudaStream_t)stream);
 }
 
 AHV_API int ahv_score_backward_saved(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
@@ -416,11 +419,12 @@ AHV_API int ahv_score_backward_saved(const float* vol_src, const float* tgt_feat
   if (!aligned16(h1_saved)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
+  const Scored p{vol_src, AHV_VOL_F32, W1, W2, b2, base, R, r_per_pair != 0, B, N};
   if (math_mode == AHV_MATH_TC)
-    return launch_score_bwd_tc(vol_src, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, grad_scores, h1_saved,
-                               pair_inv_scale, grad_vol, grad_tgt, grad_W1, grad_W2, grad_b2, B, N, (cudaStream_t)stream);
-  return launch_score_bwd(vol_src, tgt_feat, R, r_per_pair != 0, W1, W2, b2, base, grad_scores, grad_vol, grad_tgt,
-                          grad_W1, grad_W2, grad_b2, B, N, (cudaStream_t)stream, h1_saved, pair_inv_scale);
+    return launch_score_bwd_tc(p, tgt_feat, grad_scores, h1_saved, pair_inv_scale, grad_vol, grad_tgt, grad_W1, grad_W2,
+                               grad_b2, (cudaStream_t)stream);
+  return launch_score_bwd(p, tgt_feat, grad_scores, grad_vol, grad_tgt, grad_W1, grad_W2, grad_b2, (cudaStream_t)stream,
+                          h1_saved, pair_inv_scale);
 }
 
 AHV_API int ahv_forward_3d2d(const float* vol, const float* W1, const float* W2, const float* b2,
@@ -432,17 +436,17 @@ AHV_API int ahv_forward_3d2d(const float* vol, const float* W1, const float* W2,
 }
 
 AHV_API size_t ahv_workspace_bytes(int B, int64_t N, int k) {
-  return B < 0 || N < 0 ? 0 : VerifyWs(B, N, k).total;
+  return B < 0 || N < 0 ? 0 : VerifyWs(nullptr, B, N, k).total;
 }
 
 AHV_API int ahv_verify_screen_stats(const void* workspace, int B, int64_t N, int* is_screened, int* flagged_pairs,
                                     int* contenders, float* max_err) {
   if (B < 0 || !n_ok(N) || !is_screened) return AHV_EINVAL;
-  const VerifyWs w(B, N, 1);
+  const VerifyWs w(const_cast<void*>(workspace), B, N, 1);
   *is_screened = screened(w, AHV_VOL_F32, AHV_MATH_TC, nullptr, 1, B, N);
   if (!*is_screened || (!flagged_pairs && !contenders && !max_err)) return AHV_OK;
   if (!workspace) return AHV_EINVAL;
-  const ScreenLists L(static_cast<unsigned char*>(const_cast<void*>(workspace)) + w.topk, B);
+  const ScreenLists& L = w.screen;
   if (flagged_pairs) AHV_CUDA_OK(cudaMemcpy(flagged_pairs, L.flagged, sizeof(int), cudaMemcpyDeviceToHost));
   if (contenders) AHV_CUDA_OK(cudaMemcpy(contenders, L.count, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost));
   if (max_err) AHV_CUDA_OK(cudaMemcpy(max_err, L.err, (size_t)B * sizeof(float), cudaMemcpyDeviceToHost));
@@ -490,9 +494,9 @@ AHV_API int ahv_score(const void* vol_src, int vol_dtype, const float* tgt_feat,
   int st = check_device();
   if (st != AHV_OK) return st;
   if ((int64_t)B * N == 0) return AHV_OK;
-  if (!workspace || workspace_bytes < VerifyWs(B, N, k).lists) return AHV_EWORKSPACE;
-  return score_chain(vol_src, vol_dtype, tgt_feat, R, r_per_pair, W1, W2, b2, base, scores, topk_val, topk_idx, k, idx_offset,
-                     B, N, math_mode, static_cast<unsigned char*>(workspace), (cudaStream_t)stream);
+  if (!workspace || workspace_bytes < VerifyWs(nullptr, B, N, k).score_bytes) return AHV_EWORKSPACE;
+  const Scored p{vol_src, vol_dtype, W1, W2, b2, base, R, r_per_pair != 0, B, N};
+  return score_chain(p, tgt_feat, scores, topk_val, topk_idx, k, idx_offset, math_mode, workspace, (cudaStream_t)stream);
 }
 
 AHV_API int ahv_verify(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
@@ -505,14 +509,15 @@ AHV_API int ahv_verify(const void* vol_src, int vol_dtype, const float* vol_tgt,
   int st = check_device();
   if (st != AHV_OK) return st;
   if ((int64_t)B * N == 0) return AHV_OK;
-  if (!workspace || workspace_bytes < VerifyWs(B, N, k).total) return AHV_EWORKSPACE;
-  return verify_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, scores, topk_val, topk_idx, R_best, k,
-                      idx_offset, B, N, math_mode, workspace, workspace_bytes, (cudaStream_t)stream, nullptr);
+  if (!workspace || workspace_bytes < VerifyWs(nullptr, B, N, k).total) return AHV_EWORKSPACE;
+  const Scored p{vol_src, vol_dtype, W1, W2, b2, base, R, r_per_pair != 0, B, N};
+  return verify_chain(p, vol_tgt, scores, topk_val, topk_idx, R_best, k, idx_offset, math_mode, workspace,
+                      (cudaStream_t)stream, nullptr);
 }
 
 // ---- two-pass selection: dense set -> top-k -> local refinement (BASELINE config 4; extension) -----------
 AHV_API size_t ahv_refine_workspace_bytes(int B, int64_t N, int k, int m) {
-  return B < 0 || N < 0 || !k_ok(k) || m < 1 ? 0 : RefineWs(B, N, k, m).total;
+  return B < 0 || N < 0 || !k_ok(k) || m < 1 ? 0 : RefineWs(nullptr, B, N, k, m).total;
 }
 
 AHV_API int ahv_refine(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R, int r_per_pair,
@@ -523,7 +528,7 @@ AHV_API int ahv_refine(const void* vol_src, int vol_dtype, const float* vol_tgt,
   if (B < 1 || N < 1 || !k_ok(k) || k > N || m < 1 || !n_ok((int64_t)k * m)) return AHV_EINVAL;
   if (!all_set(first_val, first_idx, first_R, cand, best_val, best_idx, workspace)) return AHV_EINVAL;
   if (!aligned16(cand)) return AHV_EINVAL;
-  const RefineWs w(B, N, k, m);
+  const RefineWs w(workspace, B, N, k, m);
   if (workspace_bytes < w.total) return AHV_EWORKSPACE;
   if (!n_ok(N) || !vol_dtype_ok(vol_dtype) || !math_mode_ok(math_mode)) return AHV_EINVAL;
   if (!all_set(vol_src, vol_tgt, R, W1, W2, b2, base)) return AHV_EINVAL;
@@ -532,17 +537,16 @@ AHV_API int ahv_refine(const void* vol_src, int vol_dtype, const float* vol_tgt,
   int st = check_device();
   if (st != AHV_OK) return st;
   cudaStream_t s = (cudaStream_t)stream;
-  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  const Scored p{vol_src, vol_dtype, W1, W2, b2, base, R, r_per_pair != 0, B, N};
   // pass 1: the whole set, top-k and their rotations
-  st = verify_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, first_val, first_idx, first_R, k, 0,
-                    B, N, math_mode, ws, w.cand, s, nullptr);
+  st = verify_chain(p, vol_tgt, nullptr, first_val, first_idx, first_R, k, 0, math_mode, w.grid, s, nullptr);
   if (st != AHV_OK) return st;
   // candidates: m rotations within max_angle_deg of each of the B*k winners (index 0 = the winner itself)
   st = launch_so3_perturb(first_R, (int64_t)B * k, m, max_angle_deg, seed, cand, s);
   if (st != AHV_OK) return st;
   // pass 2: per-pair candidate sets [B, k*m], arg-max
-  return verify_chain(vol_src, vol_dtype, vol_tgt, cand, 1, W1, W2, b2, base, nullptr, best_val, best_idx, R_best, 1, 0, B,
-                      (int64_t)k * m, math_mode, ws + w.cand, w.total - w.cand, s, nullptr);
+  return verify_chain(p.with_R(cand, true, (int64_t)k * m), vol_tgt, nullptr, best_val, best_idx, R_best, 1, 0, math_mode,
+                      w.cand, s, nullptr);
 }
 
 // ---- gradient ascent of the fp32 score on SO(3), alone and after the grid pass (extension) ---------------
@@ -561,12 +565,12 @@ AHV_API int ahv_gradient_ascent(const void* vol_src, int vol_dtype, const float*
   if (!all_aligned16(vol_src, tgt_feat, R_init, R_out, W1, W2)) return AHV_EINVAL;
   int st = check_device();
   if (st != AHV_OK) return st;
-  return launch_gradient_ascent(vol_src, vol_dtype, tgt_feat, R_init, W1, W2, b2, base, steps, step_deg, R_out, score_out,
-                                B, K, (cudaStream_t)stream);
+  const Scored p{vol_src, vol_dtype, W1, W2, b2, base, R_init, true, B, K};
+  return launch_gradient_ascent(p, tgt_feat, steps, step_deg, R_out, score_out, (cudaStream_t)stream);
 }
 
 AHV_API size_t ahv_refine_gradient_workspace_bytes(int B, int64_t N, int k) {
-  return B < 0 || N < 0 || !k_ok(k) ? 0 : ShardedRefineWs(B, N, k, 1).total;
+  return B < 0 || N < 0 || !k_ok(k) ? 0 : ShardedRefineWs(nullptr, B, N, k, 1).total;
 }
 
 namespace {
@@ -594,12 +598,12 @@ AHV_API int ahv_refine_gradient(const void* vol_src, int vol_dtype, const float*
   if (!refine_gradient_args_ok(vol_src, vol_dtype, vol_tgt, R, W1, W2, b2, base, k, steps, step_deg, 0.0f, first_val, first_idx,
                                first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode, workspace))
     return AHV_EINVAL;
-  if (workspace_bytes < ShardedRefineWs(B, N, k, 1).total) return AHV_EWORKSPACE;
+  if (workspace_bytes < ShardedRefineWs(nullptr, B, N, k, 1).total) return AHV_EWORKSPACE;
   int st = check_device();
   if (st != AHV_OK) return st;
-  return refine_gradient_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, 0.0f, first_val,
-                               first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode, workspace,
-                               (cudaStream_t)stream, nullptr, 0);
+  const Scored p{vol_src, vol_dtype, W1, W2, b2, base, R, r_per_pair != 0, B, N};
+  return refine_gradient_chain(p, vol_tgt, k, steps, step_deg, 0.0f, first_val, first_idx, first_R, R_all, score_all, best_val,
+                               best_idx, R_best, math_mode, workspace, (cudaStream_t)stream, nullptr, 0);
 }
 
 AHV_API int ahv_refine_gradient_distinct(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R,
@@ -611,36 +615,53 @@ AHV_API int ahv_refine_gradient_distinct(const void* vol_src, int vol_dtype, con
   if (!refine_gradient_args_ok(vol_src, vol_dtype, vol_tgt, R, W1, W2, b2, base, k, steps, step_deg, min_sep_deg, first_val,
                                first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode, workspace))
     return AHV_EINVAL;
-  if (workspace_bytes < ShardedRefineWs(B, N, k, 1).total) return AHV_EWORKSPACE;
+  if (workspace_bytes < ShardedRefineWs(nullptr, B, N, k, 1).total) return AHV_EWORKSPACE;
   int st = check_device();
   if (st != AHV_OK) return st;
-  return refine_gradient_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, min_sep_deg,
-                               first_val, first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode,
-                               workspace, (cudaStream_t)stream, nullptr, 0);
+  const Scored p{vol_src, vol_dtype, W1, W2, b2, base, R, r_per_pair != 0, B, N};
+  return refine_gradient_chain(p, vol_tgt, k, steps, step_deg, min_sep_deg, first_val, first_idx, first_R, R_all, score_all,
+                               best_val, best_idx, R_best, math_mode, workspace, (cudaStream_t)stream, nullptr, 0);
 }
 
 // ---- coarse-to-fine search on the nested Hopf grid (extension) --------------------------------------------
 namespace {
 constexpr int kHopfMaxBaseLevel = 6;
 
+// the result of a search of zero levels: the base level's
+int copy_base_level(const float* first_val, const int64_t* first_idx, const float* first_R, float* val, int64_t* idx,
+                    float* R_out, int B, int k, cudaStream_t s) {
+  AHV_CUDA_OK(cudaMemcpyAsync(val, first_val, (size_t)B * k * sizeof(float), cudaMemcpyDeviceToDevice, s));
+  AHV_CUDA_OK(cudaMemcpyAsync(idx, first_idx, (size_t)B * k * sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
+  AHV_CUDA_OK(cudaMemcpyAsync(R_out, first_R, (size_t)B * k * 9 * sizeof(float), cudaMemcpyDeviceToDevice, s));
+  return AHV_OK;
+}
+
 // ahv_search_hierarchical: [scoring workspace of the larger pass | target features B*32*64 fp32 | base grid n0*9 fp32
 //  | children [B,8k] int64 | their rotations [B,8k,9] fp32 | a level's top-k [B,k] fp32 and int64 | parents [B,k] int64]
 struct HierWs {
-  size_t tgt, grid, kids, kids_R, lval, lidx, par, total;
-  HierWs(int B, int base_level, int k)
-      : tgt(std::max(VerifyWs(B, hopf_cells(base_level), k).lists, VerifyWs(B, 8 * (int64_t)k, k).lists)),
-        grid(tgt + align_up((size_t)B * kO * kP * sizeof(float), 256)),
-        kids(grid + align_up((size_t)hopf_cells(base_level) * 9 * sizeof(float), 256)),
-        kids_R(kids + align_up((size_t)B * 8 * k * sizeof(int64_t), 256)),
-        lval(kids_R + align_up((size_t)B * 8 * k * 9 * sizeof(float), 256)),
-        lidx(lval + align_up((size_t)B * k * sizeof(float), 256)),
-        par(lidx + align_up((size_t)B * k * sizeof(int64_t), 256)),
-        total(par + align_up((size_t)B * k * sizeof(int64_t), 256)) {}
+  float *tgt, *grid;
+  int64_t* kids;
+  float *kids_R, *lval;
+  int64_t *lidx, *par;
+  size_t total;
+  HierWs(void* ws, int B, int base_level, int k) {
+    Carve c(ws);
+    c.take<unsigned char>(std::max(VerifyWs(nullptr, B, hopf_cells(base_level), k).score_bytes,
+                                   VerifyWs(nullptr, B, 8 * (int64_t)k, k).score_bytes), 256);
+    tgt = c.take<float>((size_t)B * kO * kP, 256);
+    grid = c.take<float>((size_t)hopf_cells(base_level) * 9, 256);
+    kids = c.take<int64_t>((size_t)B * 8 * k, 256);
+    kids_R = c.take<float>((size_t)B * 8 * k * 9, 256);
+    lval = c.take<float>((size_t)B * k, 256);
+    lidx = c.take<int64_t>((size_t)B * k, 256);
+    par = c.take<int64_t>((size_t)B * k, 256);
+    total = c.off;
+  }
 };
 }  // namespace
 
 AHV_API size_t ahv_search_hierarchical_workspace_bytes(int B, int base_level, int k) {
-  return B < 1 || base_level < 0 || base_level > kHopfMaxBaseLevel || !k_ok(k) ? 0 : HierWs(B, base_level, k).total;
+  return B < 1 || base_level < 0 || base_level > kHopfMaxBaseLevel || !k_ok(k) ? 0 : HierWs(nullptr, B, base_level, k).total;
 }
 
 AHV_API int ahv_search_hierarchical(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* W1, const float* W2,
@@ -652,67 +673,65 @@ AHV_API int ahv_search_hierarchical(const void* vol_src, int vol_dtype, const fl
   if (!all_set(vol_src, vol_tgt, W1, W2, b2, base, first_val, first_idx, first_R, val, idx, R_out, workspace))
     return AHV_EINVAL;
   if (!all_aligned16(vol_src, vol_tgt, W1, W2, first_R, R_out, workspace)) return AHV_EINVAL;
-  const HierWs w(B, base_level, k);
+  const HierWs w(workspace, B, base_level, k);
   if (workspace_bytes < w.total) return AHV_EWORKSPACE;
   int st = check_device();
   if (st != AHV_OK) return st;
   cudaStream_t s = (cudaStream_t)stream;
-  unsigned char* ws = static_cast<unsigned char*>(workspace);
-  float* tgt = reinterpret_cast<float*>(ws + w.tgt);
-  float* grid = reinterpret_cast<float*>(ws + w.grid);
-  int64_t* kids = reinterpret_cast<int64_t*>(ws + w.kids);
-  float* kids_R = reinterpret_cast<float*>(ws + w.kids_R);
-  int64_t* lidx = reinterpret_cast<int64_t*>(ws + w.lidx);
-  int64_t* par = reinterpret_cast<int64_t*>(ws + w.par);
   const int64_t n0 = hopf_cells(base_level), nc = 8 * (int64_t)k;
-  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
-  if (st == AHV_OK) st = launch_so3_hopf_grid(base_level, 0, grid, n0, s);
+  const Scored p{vol_src, vol_dtype, W1, W2, b2, base, w.grid, false, B, n0};
+  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, w.tgt, B, s);
+  if (st == AHV_OK) st = launch_so3_hopf_grid(base_level, 0, w.grid, n0, s);
   // the base level: one set shared by the B pairs; its local indices are grid indices
-  if (st == AHV_OK)
-    st = score_chain(vol_src, vol_dtype, tgt, grid, 0, W1, W2, b2, base, nullptr, first_val, first_idx, k, 0, B, n0, math_mode, ws,
-                     s);
-  if (st == AHV_OK) st = launch_gather_rotations(grid, 0, first_idx, 0, B, n0, k, first_R, s);
+  if (st == AHV_OK) st = score_chain(p, w.tgt, nullptr, first_val, first_idx, k, 0, math_mode, workspace, s);
+  if (st == AHV_OK) st = launch_gather_rotations(w.grid, 0, first_idx, 0, B, n0, k, first_R, s);
   if (st != AHV_OK) return st;
-  if (levels == 0) {
-    AHV_CUDA_OK(cudaMemcpyAsync(val, first_val, (size_t)B * k * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    AHV_CUDA_OK(cudaMemcpyAsync(idx, first_idx, (size_t)B * k * sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
-    AHV_CUDA_OK(cudaMemcpyAsync(R_out, first_R, (size_t)B * k * 9 * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    return AHV_OK;
-  }
+  if (levels == 0) return copy_base_level(first_val, first_idx, first_R, val, idx, R_out, B, k, s);
   // Each level scores the 8 children of the pair's k cells, the cells taken in ascending index order.  The candidate
   // list then ascends in grid index (the children of cell i are 8i .. 8i+7), so the top-k's tie rule (lowest local
   // index) is the lowest grid index.
-  st = launch_hopf_pick(nullptr, 0, first_idx, B, k, true, par, s);
+  st = launch_hopf_pick(nullptr, 0, first_idx, B, k, true, w.par, s);
   for (int l = 0; l < levels && st == AHV_OK; ++l) {
     const bool last = l == levels - 1;
-    st = launch_so3_hopf_children(base_level + l, par, (int64_t)B * k, kids, kids_R, s);
+    st = launch_so3_hopf_children(base_level + l, w.par, (int64_t)B * k, w.kids, w.kids_R, s);
     if (st == AHV_OK)
-      st = score_chain(vol_src, vol_dtype, tgt, kids_R, 1, W1, W2, b2, base, nullptr,
-                       last ? val : reinterpret_cast<float*>(ws + w.lval), lidx, k, 0, B, nc, math_mode, ws, s);
-    if (st == AHV_OK) st = launch_hopf_pick(kids, nc, lidx, B, k, !last, last ? idx : par, s);
+      st = score_chain(p.with_R(w.kids_R, true, nc), w.tgt, nullptr, last ? val : w.lval, w.lidx, k, 0, math_mode, workspace,
+                       s);
+    if (st == AHV_OK) st = launch_hopf_pick(w.kids, nc, w.lidx, B, k, !last, last ? idx : w.par, s);
   }
   if (st != AHV_OK) return st;
-  return launch_gather_rotations(kids_R, 1, lidx, 0, B, nc, k, R_out, s);
+  return launch_gather_rotations(w.kids_R, 1, w.lidx, 0, B, nc, k, R_out, s);
 }
 
 // ---- coarse-to-fine search that keeps k distinct modes (extension) ------------------------------------------------
 namespace {
 constexpr int kMaxBeam = 8;
 
-// ahv_search_modes: [scoring workspace of the larger pass (its score region holds the base scores until the first level)
-//  | target features B*32*64 fp32 | base grid n0*9 fp32 | base slots B*n0 bytes | children [B,8kw] int64 | their rotations
-//  [B,8kw,9] fp32 | beams [B,k,w] int64 | the beams for the children generator [B,k,w] int64]
+// ahv_search_modes: [scoring workspace of the larger pass | target features B*32*64 fp32 | base grid n0*9 fp32 | base
+//  slots B*n0 bytes | children [B,8kw] int64 | their rotations [B,8kw,9] fp32 | beams [B,k,w] int64 | the beams for the
+//  children generator [B,k,w] int64].  `scores`, the scoring workspace's score region, holds the base scores until the
+//  first level.
 struct ModesWs {
-  size_t tgt, grid, slot, kids, kids_R, par, gen, total;
-  ModesWs(int B, int base_level, int k, int w)
-      : tgt(std::max(VerifyWs(B, hopf_cells(base_level), 0).lists, VerifyWs(B, 8 * (int64_t)k * w, 0).lists)),
-        grid(tgt + align_up((size_t)B * kO * kP * sizeof(float), 256)),
-        slot(grid + align_up((size_t)hopf_cells(base_level) * 9 * sizeof(float), 256)),
-        kids(slot + align_up((size_t)B * hopf_cells(base_level), 256)),
-        kids_R(kids + align_up((size_t)B * 8 * k * w * sizeof(int64_t), 256)),
-        par(kids_R + align_up((size_t)B * 8 * k * w * 9 * sizeof(float), 256)),
-        gen(par + align_up((size_t)B * k * w * sizeof(int64_t), 256)),
-        total(gen + align_up((size_t)B * k * w * sizeof(int64_t), 256)) {}
+  float *scores, *tgt, *grid;
+  uint8_t* slot;
+  int64_t* kids;
+  float* kids_R;
+  int64_t *par, *gen;
+  size_t total;
+  ModesWs(void* ws, int B, int base_level, int k, int w) {
+    const int64_t n0 = hopf_cells(base_level), nc = 8 * (int64_t)k * w;
+    Carve c(ws);
+    scores = VerifyWs(ws, B, n0, 0).scores;
+    c.take<unsigned char>(std::max(VerifyWs(nullptr, B, n0, 0).score_bytes, VerifyWs(nullptr, B, nc, 0).score_bytes), 256);
+    tgt = c.take<float>((size_t)B * kO * kP, 256);
+    grid = c.take<float>((size_t)n0 * 9, 256);
+    slot = c.take<uint8_t>((size_t)B * n0, 256);
+    kids = c.take<int64_t>((size_t)B * nc, 256);
+    kids_R = c.take<float>((size_t)B * nc * 9, 256);
+    par = c.take<int64_t>((size_t)B * k * w, 256);
+    gen = c.take<int64_t>((size_t)B * k * w, 256);
+    total = c.off;
+  }
 };
 
 bool modes_sizes_ok(int B, int base_level, int k, int beam) {
@@ -721,7 +740,7 @@ bool modes_sizes_ok(int B, int base_level, int k, int beam) {
 }  // namespace
 
 AHV_API size_t ahv_search_modes_workspace_bytes(int B, int base_level, int k, int beam) {
-  return modes_sizes_ok(B, base_level, k, beam) ? ModesWs(B, base_level, k, beam).total : 0;
+  return modes_sizes_ok(B, base_level, k, beam) ? ModesWs(nullptr, B, base_level, k, beam).total : 0;
 }
 
 AHV_API int ahv_search_modes(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* W1, const float* W2,
@@ -734,42 +753,28 @@ AHV_API int ahv_search_modes(const void* vol_src, int vol_dtype, const float* vo
   if (!all_set(vol_src, vol_tgt, W1, W2, b2, base, first_val, first_idx, first_R, val, idx, R_out, workspace))
     return AHV_EINVAL;
   if (!all_aligned16(vol_src, vol_tgt, W1, W2, first_R, R_out, workspace)) return AHV_EINVAL;
-  const ModesWs w(B, base_level, k, beam);
+  const ModesWs w(workspace, B, base_level, k, beam);
   if (workspace_bytes < w.total) return AHV_EWORKSPACE;
   int st = check_device();
   if (st != AHV_OK) return st;
   cudaStream_t s = (cudaStream_t)stream;
-  unsigned char* ws = static_cast<unsigned char*>(workspace);
-  float* tgt = reinterpret_cast<float*>(ws + w.tgt);
-  float* grid = reinterpret_cast<float*>(ws + w.grid);
-  int64_t* kids = reinterpret_cast<int64_t*>(ws + w.kids);
-  float* kids_R = reinterpret_cast<float*>(ws + w.kids_R);
-  int64_t* par = reinterpret_cast<int64_t*>(ws + w.par);
-  int64_t* gen = reinterpret_cast<int64_t*>(ws + w.gen);
-  const float* sc = reinterpret_cast<const float*>(ws);  // score_chain's score region when it is given none
   const int64_t n0 = hopf_cells(base_level), nc = 8 * (int64_t)k * beam;
-  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, tgt, B, s);
-  if (st == AHV_OK) st = launch_so3_hopf_grid(base_level, 0, grid, n0, s);
+  const Scored p{vol_src, vol_dtype, W1, W2, b2, base, w.grid, false, B, n0};
+  st = launch_forward_3d2d(vol_tgt, W1, W2, b2, w.tgt, B, s);
+  if (st == AHV_OK) st = launch_so3_hopf_grid(base_level, 0, w.grid, n0, s);
   // the base level (one set shared by the B pairs; local indices are grid indices) and its k distinct winners
-  if (st == AHV_OK)
-    st = score_chain(vol_src, vol_dtype, tgt, grid, 0, W1, W2, b2, base, nullptr, nullptr, nullptr, 0, 0, B, n0, math_mode, ws,
-                     s);
-  if (st == AHV_OK) st = launch_topk_distinct(sc, grid, 0, B, n0, k, min_sep_deg, first_val, first_idx, first_R, s);
+  if (st == AHV_OK) st = score_chain(p, w.tgt, nullptr, nullptr, nullptr, 0, 0, math_mode, workspace, s);
+  if (st == AHV_OK) st = launch_topk_distinct(w.scores, w.grid, 0, B, n0, k, min_sep_deg, first_val, first_idx, first_R, s);
   if (st != AHV_OK) return st;
-  if (levels == 0) {
-    AHV_CUDA_OK(cudaMemcpyAsync(val, first_val, (size_t)B * k * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    AHV_CUDA_OK(cudaMemcpyAsync(idx, first_idx, (size_t)B * k * sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
-    AHV_CUDA_OK(cudaMemcpyAsync(R_out, first_R, (size_t)B * k * 9 * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    return AHV_OK;
-  }
-  st = launch_modes_beams(sc, grid, n0, first_idx, first_R, B, k, beam, min_sep_deg, ws + w.slot, par, gen, s);
+  if (levels == 0) return copy_base_level(first_val, first_idx, first_R, val, idx, R_out, B, k, s);
+  st = launch_modes_beams(w.scores, w.grid, n0, first_idx, first_R, B, k, beam, min_sep_deg, w.slot, w.par, w.gen, s);
   // each level scores the children of every beam as a per-pair set [B, 8kw] and keeps each slot's top-w
   for (int l = 0; l < levels && st == AHV_OK; ++l) {
-    st = launch_so3_hopf_children(base_level + l, gen, (int64_t)B * k * beam, kids, kids_R, s);
+    st = launch_so3_hopf_children(base_level + l, w.gen, (int64_t)B * k * beam, w.kids, w.kids_R, s);
     if (st == AHV_OK)
-      st = score_chain(vol_src, vol_dtype, tgt, kids_R, 1, W1, W2, b2, base, nullptr, nullptr, nullptr, 0, 0, B, nc, math_mode,
-                       ws, s);
-    if (st == AHV_OK) st = launch_modes_level(sc, kids, kids_R, B, k, beam, l == levels - 1, par, gen, val, idx, R_out, s);
+      st = score_chain(p.with_R(w.kids_R, true, nc), w.tgt, nullptr, nullptr, nullptr, 0, 0, math_mode, workspace, s);
+    if (st == AHV_OK)
+      st = launch_modes_level(w.scores, w.kids, w.kids_R, B, k, beam, l == levels - 1, w.par, w.gen, val, idx, R_out, s);
   }
   return st;
 }
@@ -963,9 +968,10 @@ AHV_API int ahv_verify_sharded(const void* vol_src, int vol_dtype, const float* 
   st = check_device();
   if (st != AHV_OK) return st;
   if (world == 1 && N == 0) return AHV_EINVAL;
-  if (!workspace || workspace_bytes < VerifyWs(B, N, k).total) return AHV_EWORKSPACE;
-  return verify_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, nullptr, topk_val, topk_idx, R_best, k,
-                      idx_offset, B, N, math_mode, workspace, workspace_bytes, (cudaStream_t)stream, &pa);
+  if (!workspace || workspace_bytes < VerifyWs(nullptr, B, N, k).total) return AHV_EWORKSPACE;
+  const Scored p{vol_src, vol_dtype, W1, W2, b2, base, R, r_per_pair != 0, B, N};
+  return verify_chain(p, vol_tgt, nullptr, topk_val, topk_idx, R_best, k, idx_offset, math_mode, workspace,
+                      (cudaStream_t)stream, &pa);
 }
 
 AHV_API int ahv_scores_exchange(const float* part, int B, int64_t N, float* scores, int rank, int world, void* const* peers,
@@ -985,7 +991,7 @@ AHV_API int ahv_scores_exchange(const float* part, int B, int64_t N, float* scor
 
 AHV_API size_t ahv_refine_gradient_sharded_workspace_bytes(int B, int64_t N, int k, int world) {
   if (B < 0 || N < 0 || !k_ok(k) || world < 1 || world > peer::kMaxPeers) return 0;
-  return ShardedRefineWs(B, N, k, world).total;
+  return ShardedRefineWs(nullptr, B, N, k, world).total;
 }
 
 AHV_API int ahv_refine_gradient_sharded(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R,
@@ -1003,12 +1009,12 @@ AHV_API int ahv_refine_gradient_sharded(const void* vol_src, int vol_dtype, cons
   if (st != AHV_OK) return st;
   if (world > 1 && (B > peer_max_pairs || k > peer_max_k)) return AHV_EINVAL;  // the slot gather's entries
   if (world > 1 && min_sep_deg > 0.0f && (!n_ok(peer_max_hyps) || N > peer_max_hyps)) return AHV_EINVAL;  // the score region
-  if (workspace_bytes < ShardedRefineWs(B, N, k, world).total) return AHV_EWORKSPACE;
+  if (workspace_bytes < ShardedRefineWs(nullptr, B, N, k, world).total) return AHV_EWORKSPACE;
   st = check_device();
   if (st != AHV_OK) return st;
-  return refine_gradient_chain(vol_src, vol_dtype, vol_tgt, R, r_per_pair, W1, W2, b2, base, k, steps, step_deg, min_sep_deg,
-                               first_val, first_idx, first_R, R_all, score_all, best_val, best_idx, R_best, B, N, math_mode,
-                               workspace, (cudaStream_t)stream, &pa, peer_max_hyps);
+  const Scored p{vol_src, vol_dtype, W1, W2, b2, base, R, r_per_pair != 0, B, N};
+  return refine_gradient_chain(p, vol_tgt, k, steps, step_deg, min_sep_deg, first_val, first_idx, first_R, R_all, score_all,
+                               best_val, best_idx, R_best, math_mode, workspace, (cudaStream_t)stream, &pa, peer_max_hyps);
 }
 
 // ---- host-buffer entries -------------------------------------------------------------------------------
@@ -1018,6 +1024,31 @@ struct ahv_host_session {
   unsigned char* d = nullptr;
   size_t bytes = 0;
   int device = -1;
+};
+
+// The device block of a host-buffer call: [source volumes | target volumes | rotations | W1, W2, b2 and base (8 floats) |
+// top-k indices, values and rotations | verification workspace]
+struct HostBlock {
+  void* src;
+  float *tgt, *R, *W1;  // W1 [32,384], then W2 [32,32], b2 [32] and base [8]
+  int64_t* idx;
+  float *val, *R_best;
+  void* ws;
+  size_t ws_bytes, total;
+  HostBlock(void* p, size_t src_b, size_t tgt_b, size_t r_b, int B, int64_t N, int k) {
+    Carve c(p);
+    src = c.take<unsigned char>(src_b, 256);
+    tgt = c.take<float>(tgt_b / sizeof(float), 256);
+    R = c.take<float>(r_b / sizeof(float), 256);
+    W1 = c.take<float>(kO * kK + kO * kO + kO + 8, 256);
+    Carve out(c.take<unsigned char>((size_t)B * k * (sizeof(int64_t) + sizeof(float) + 9 * sizeof(float)), 256));
+    idx = out.take<int64_t>((size_t)B * k, 1);
+    val = out.take<float>((size_t)B * k, 1);
+    R_best = out.take<float>((size_t)B * k * 9, 1);
+    ws_bytes = VerifyWs(nullptr, B, N, k).total;
+    ws = c.take<unsigned char>(ws_bytes, 1);
+    total = c.off;
+  }
 };
 
 AHV_API int ahv_host_session_create(ahv_host_session** session) {
@@ -1057,58 +1088,43 @@ AHV_API int ahv_predict_host_ex(ahv_host_session* session, const void* vol_src_h
   const size_t src_b = (size_t)B * kC * kVox * (vol_dtype == AHV_VOL_BF16 ? 2 : 4);
   const size_t tgt_b = (size_t)B * kC * kVox * sizeof(float);
   const size_t r_b = (size_t)(r_per_pair ? B : 1) * N * 9 * sizeof(float);
-  const size_t w_b = (size_t)(kO * kK + kO * kO + kO + 8) * sizeof(float);
-  const size_t out_b = (size_t)B * k * (sizeof(float) + sizeof(int64_t) + 9 * sizeof(float));
-  const size_t ws_b = VerifyWs(B, N, k).total;
-  const size_t total = align_up(src_b, 256) + align_up(tgt_b, 256) + align_up(r_b, 256) + align_up(w_b, 256) +
-                       align_up(out_b, 256) + ws_b;
-  if (session->bytes < total) {  // grow (rare): the stream may still use the old block
+  const HostBlock nb(nullptr, src_b, tgt_b, r_b, B, N, k);
+  if (session->bytes < nb.total) {  // grow (rare): the stream may still use the old block
     if (cudaStreamSynchronize(s) != cudaSuccess) return AHV_ECUDA;
     if (session->d && cudaFree(session->d) != cudaSuccess) return AHV_ECUDA;
     session->d = nullptr;
     session->bytes = 0;
-    if (cudaMalloc((void**)&session->d, total) != cudaSuccess) return AHV_ECUDA;
-    session->bytes = total;
+    if (cudaMalloc((void**)&session->d, nb.total) != cudaSuccess) return AHV_ECUDA;
+    session->bytes = nb.total;
   }
-  unsigned char* p = session->d;
-  auto take = [&](size_t bytes) { unsigned char* r = p; p += align_up(bytes, 256); return r; };
-  void* d_src = take(src_b);
-  float* d_tgt = (float*)take(tgt_b);
-  float* d_R = (float*)take(r_b);
-  float* d_w = (float*)take(w_b);
-  unsigned char* d_out = take(out_b);
-  void* d_ws = p;
-  float* d_W1 = d_w; float* d_W2 = d_W1 + kO * kK; float* d_b2 = d_W2 + kO * kO; float* d_base = d_b2 + kO;
-  // d_out: [idx int64 B*k | val fp32 B*k | R_best fp32 B*k*9]
-  int64_t* d_idx = (int64_t*)d_out;
-  float* d_val = (float*)(d_out + (size_t)B * k * sizeof(int64_t));
-  float* d_Rb = d_val + (size_t)B * k;
+  const HostBlock d(session->d, src_b, tgt_b, r_b, B, N, k);
+  float* d_W1 = d.W1; float* d_W2 = d_W1 + kO * kK; float* d_b2 = d_W2 + kO * kO; float* d_base = d_b2 + kO;
   st = AHV_ECUDA;
   do {
-    if (cudaMemcpyAsync(d_src, vol_src_host, src_b, cudaMemcpyHostToDevice, s) != cudaSuccess) break;
-    if (cudaMemcpyAsync(d_tgt, vol_tgt_host, tgt_b, cudaMemcpyHostToDevice, s) != cudaSuccess) break;
-    if (cudaMemcpyAsync(d_R, R_host, r_b, cudaMemcpyHostToDevice, s) != cudaSuccess) break;
+    if (cudaMemcpyAsync(d.src, vol_src_host, src_b, cudaMemcpyHostToDevice, s) != cudaSuccess) break;
+    if (cudaMemcpyAsync(d.tgt, vol_tgt_host, tgt_b, cudaMemcpyHostToDevice, s) != cudaSuccess) break;
+    if (cudaMemcpyAsync(d.R, R_host, r_b, cudaMemcpyHostToDevice, s) != cudaSuccess) break;
     if (cudaMemcpyAsync(d_W1, W1_host, kO * kK * 4, cudaMemcpyHostToDevice, s) != cudaSuccess) break;
     if (cudaMemcpyAsync(d_W2, W2_host, kO * kO * 4, cudaMemcpyHostToDevice, s) != cudaSuccess) break;
     if (cudaMemcpyAsync(d_b2, b2_host, kO * 4, cudaMemcpyHostToDevice, s) != cudaSuccess) break;
     if (cudaMemcpyAsync(d_base, base_host, 8 * 4, cudaMemcpyHostToDevice, s) != cudaSuccess) break;
     if (world > 1)
-      st = ahv_verify_sharded(d_src, vol_dtype, d_tgt, d_R, r_per_pair, d_W1, d_W2, d_b2, d_base, d_val, d_idx, d_Rb, k,
-                              idx_offset, B, N, math_mode, d_ws, ws_b, rank, world, peers, peer_max_pairs, peer_max_k,
+      st = ahv_verify_sharded(d.src, vol_dtype, d.tgt, d.R, r_per_pair, d_W1, d_W2, d_b2, d_base, d.val, d.idx, d.R_best, k,
+                              idx_offset, B, N, math_mode, d.ws, d.ws_bytes, rank, world, peers, peer_max_pairs, peer_max_k,
                               stream);
     else
-      st = ahv_verify(d_src, vol_dtype, d_tgt, d_R, r_per_pair, d_W1, d_W2, d_b2, d_base,
-                      scores_host ? (float*)d_ws : nullptr, d_val, d_idx, d_Rb, k, idx_offset, B, N, math_mode, d_ws, ws_b,
+      st = ahv_verify(d.src, vol_dtype, d.tgt, d.R, r_per_pair, d_W1, d_W2, d_b2, d_base,
+                      scores_host ? (float*)d.ws : nullptr, d.val, d.idx, d.R_best, k, idx_offset, B, N, math_mode, d.ws, d.ws_bytes,
                       stream);
     if (st != AHV_OK) break;
     st = AHV_ECUDA;
     if (scores_host &&
-        cudaMemcpyAsync(scores_host, d_ws, (size_t)B * N * 4, cudaMemcpyDeviceToHost, s) != cudaSuccess)
+        cudaMemcpyAsync(scores_host, d.ws, (size_t)B * N * 4, cudaMemcpyDeviceToHost, s) != cudaSuccess)
       break;
-    if (cudaMemcpyAsync(topk_idx_host, d_idx, (size_t)B * k * 8, cudaMemcpyDeviceToHost, s) != cudaSuccess) break;
-    if (cudaMemcpyAsync(topk_val_host, d_val, (size_t)B * k * 4, cudaMemcpyDeviceToHost, s) != cudaSuccess) break;
+    if (cudaMemcpyAsync(topk_idx_host, d.idx, (size_t)B * k * 8, cudaMemcpyDeviceToHost, s) != cudaSuccess) break;
+    if (cudaMemcpyAsync(topk_val_host, d.val, (size_t)B * k * 4, cudaMemcpyDeviceToHost, s) != cudaSuccess) break;
     if (R_best_host &&
-        cudaMemcpyAsync(R_best_host, d_Rb, (size_t)B * k * 36, cudaMemcpyDeviceToHost, s) != cudaSuccess)
+        cudaMemcpyAsync(R_best_host, d.R_best, (size_t)B * k * 36, cudaMemcpyDeviceToHost, s) != cudaSuccess)
       break;
     st = AHV_OK;
   } while (0);

@@ -152,33 +152,31 @@ ascent_fp32_kernel(const T* __restrict__ vol_src, const float* __restrict__ tgt_
 }
 
 template <bool kItemRange>
-void launch_ascent(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R_init, const float* W1,
-                   const float* W2, const float* b2, const float* base, int steps, float theta0, float* R_out,
-                   float* score_out, int B, int K, const int64_t* skip_idx, int64_t item_lo, int64_t item_hi,
-                   unsigned grid, size_t smem, cudaStream_t s, cudaError_t* err) {
-  if (vol_dtype == AHV_VOL_F32) {
+void launch_ascent(const Scored& p, const float* tgt_feat, int steps, float theta0, float* R_out, float* score_out,
+                   const int64_t* skip_idx, int64_t item_lo, int64_t item_hi, unsigned grid, size_t smem, cudaStream_t s,
+                   cudaError_t* err) {
+  const int K = (int)p.N;
+  if (p.vol_dtype == AHV_VOL_F32) {
     *err = cudaFuncSetAttribute(ascent_fp32_kernel<float, kItemRange>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (*err != cudaSuccess) return;
-    ascent_fp32_kernel<float, kItemRange><<<grid, kThreads, smem, s>>>((const float*)vol_src, tgt_feat, R_init, W1, W2, b2,
-                                                                       base, steps, theta0, R_out, score_out, B, K, skip_idx,
+    ascent_fp32_kernel<float, kItemRange><<<grid, kThreads, smem, s>>>(p.vol_f32(), tgt_feat, p.R, p.W1, p.W2, p.b2, p.base,
+                                                                       steps, theta0, R_out, score_out, p.B, K, skip_idx,
                                                                        item_lo, item_hi);
   } else {
     *err = cudaFuncSetAttribute(ascent_fp32_kernel<__nv_bfloat16, kItemRange>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)smem);
     if (*err != cudaSuccess) return;
-    ascent_fp32_kernel<__nv_bfloat16, kItemRange><<<grid, kThreads, smem, s>>>((const __nv_bfloat16*)vol_src, tgt_feat, R_init,
-                                                                               W1, W2, b2, base, steps, theta0, R_out,
-                                                                               score_out, B, K, skip_idx, item_lo, item_hi);
+    ascent_fp32_kernel<__nv_bfloat16, kItemRange><<<grid, kThreads, smem, s>>>((const __nv_bfloat16*)p.vol_src, tgt_feat, p.R,
+                                                                               p.W1, p.W2, p.b2, p.base, steps, theta0, R_out,
+                                                                               score_out, p.B, K, skip_idx, item_lo, item_hi);
   }
   *err = cudaGetLastError();
 }
 
-int launch_gradient_ascent(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R_init, const float* W1,
-                           const float* W2, const float* b2, const float* base, int steps, float step_deg, float* R_out,
-                           float* score_out, int B, int K, cudaStream_t s, const int64_t* skip_idx, int64_t item_lo,
-                           int64_t item_hi) {
+int launch_gradient_ascent(const Scored& p, const float* tgt_feat, int steps, float step_deg, float* R_out,
+                           float* score_out, cudaStream_t s, const int64_t* skip_idx, int64_t item_lo, int64_t item_hi) {
   const bool ranged = item_hi >= 0;
-  const int64_t total = ranged ? item_hi - item_lo : (int64_t)B * K;
+  const int64_t total = ranged ? item_hi - item_lo : (int64_t)p.B * p.N;
   if (total <= 0) return AHV_OK;
   int dev = 0, sms = 0;
   AHV_CUDA_OK(cudaGetDevice(&dev));
@@ -188,11 +186,9 @@ int launch_gradient_ascent(const void* vol_src, int vol_dtype, const float* tgt_
   const float theta0 = (float)((double)step_deg * (3.14159265358979323846 / 180.0));  // math.radians, rounded once
   cudaError_t err = cudaSuccess;
   if (ranged)
-    launch_ascent<true>(vol_src, vol_dtype, tgt_feat, R_init, W1, W2, b2, base, steps, theta0, R_out, score_out, B, K, skip_idx,
-                        item_lo, item_hi, grid, smem, s, &err);
+    launch_ascent<true>(p, tgt_feat, steps, theta0, R_out, score_out, skip_idx, item_lo, item_hi, grid, smem, s, &err);
   else
-    launch_ascent<false>(vol_src, vol_dtype, tgt_feat, R_init, W1, W2, b2, base, steps, theta0, R_out, score_out, B, K, skip_idx,
-                         0, 0, grid, smem, s, &err);
+    launch_ascent<false>(p, tgt_feat, steps, theta0, R_out, score_out, skip_idx, 0, 0, grid, smem, s, &err);
   AHV_CUDA_OK(err);
   return AHV_OK;
 }

@@ -130,6 +130,46 @@ inline int sm_count() {
 
 namespace peer { struct Args; }  // ahv_peer.cuh
 
+// A cursor that places workspace regions one after another from `base`, each padded to a multiple of `align` bytes,
+// and hands out typed pointers.  With a null base it only counts bytes: `off` is then the size of the layout so far.
+struct Carve {
+  unsigned char* base;
+  size_t off = 0;
+  explicit Carve(void* p = nullptr) : base(static_cast<unsigned char*>(p)) {}
+  template <class T> T* take(size_t n, size_t align) {
+    T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
+    off += (n * sizeof(T) + align - 1) / align * align;
+    return p;
+  }
+};
+// the size of layout L (a struct constructed from a Carve and the sizes `a`)
+template <class L, class... A> size_t bytes_of(A... a) {
+  Carve c;
+  (void)L(c, a...);
+  return c.off;
+}
+
+// What every scorer reads: B pairs of source volumes (vol_dtype: AHV_VOL_*), the head, and N rotations per pair
+// (R [N][9] shared by the pairs, or [B][N][9] when r_per_pair).
+struct Scored {
+  const void* vol_src;
+  int vol_dtype;
+  const float *W1, *W2, *b2, *base;
+  const float* R;
+  bool r_per_pair;
+  int B;
+  int64_t N;
+  // the same pairs and head with another rotation set
+  Scored with_R(const float* R_, bool per_pair, int64_t N_) const {
+    Scored p = *this;
+    p.R = R_;
+    p.r_per_pair = per_pair;
+    p.N = N_;
+    return p;
+  }
+  const float* vol_f32() const { return static_cast<const float*>(vol_src); }
+};
+
 // Launch-side helpers implemented in the .cu files --------------------------
 int launch_so3_from_normals(const float* normals, float* R, int64_t n, cudaStream_t s);
 int launch_so3_sample(uint64_t seed, int64_t first, float* R, int64_t n, cudaStream_t s);
@@ -151,18 +191,15 @@ int launch_rotate_volume_bwd(const float* grad_out, int per_rot, const float* R,
                              float* grad_vol, int64_t n, cudaStream_t s);
 int launch_rotate_volume_grad_R(const float* vol, int per_rot, const float* R, const float* base, const float* grad_out,
                                 float* grad_R, int64_t n, cudaStream_t s);
-// The fused backward kernels (ahv_score_bwd.cu, ahv_score_bwd_tc.cu) on `grid` CTAs, 0: one per SM (at most one per
-// item).  det: the deterministic instance, whose outputs are the workspace slots below (launch_score_bwd_det).
-int launch_score_bwd(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
-                     const float* W1, const float* W2, const float* b2, const float* base,
-                     const float* grad_scores, float* g_vol, float* g_tgt, float* g_W1, float* g_W2,
-                     float* g_b2, int B, int64_t N, cudaStream_t s, const void* h1_saved = nullptr,
+// The fused backward kernels (ahv_score_bwd.cu, ahv_score_bwd_tc.cu; fp32 source volumes) on `grid` CTAs, 0: one per SM
+// (at most one per item).  det: the deterministic instance, whose outputs are the workspace slots below
+// (launch_score_bwd_det).
+int launch_score_bwd(const Scored& p, const float* tgt_feat, const float* grad_scores, float* g_vol, float* g_tgt,
+                     float* g_W1, float* g_W2, float* g_b2, cudaStream_t s, const void* h1_saved = nullptr,
                      const float* pair_inv = nullptr, float* g_R = nullptr, unsigned grid = 0, bool det = false);
-int launch_score_bwd_tc(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
-                        const float* W1, const float* W2, const float* b2, const float* base,
-                        const float* grad_scores, const void* h1_saved, const float* pair_inv, float* g_vol,
-                        float* g_tgt, float* g_W1, float* g_W2, float* g_b2, int B, int64_t N, cudaStream_t s,
-                        unsigned grid = 0, bool det = false);
+int launch_score_bwd_tc(const Scored& p, const float* tgt_feat, const float* grad_scores, const void* h1_saved,
+                        const float* pair_inv, float* g_vol, float* g_tgt, float* g_W1, float* g_W2, float* g_b2,
+                        cudaStream_t s, unsigned grid = 0, bool det = false);
 // Deterministic backward (ahv_score_backward_det).  The kernels store what the atomic instances add into global memory
 // in per-CTA workspace slots, and score_bwd_det_reduce adds the slots of every output element in increasing slot order.
 //   weight slot c (one per CTA, c < grid):   dW1 [32][384] | dW2 [32][32] | db2 [32]              kDetWSlot floats
@@ -173,52 +210,82 @@ int launch_score_bwd_tc(const float* vol_src, const float* tgt_feat, const float
 constexpr int kDetGridCap = 160;
 constexpr int kDetWSlot = kO * kK + kO * kO + kO;
 constexpr int kDetSegSlot = kC * kVox + kO * kP;
-struct DetBwdWs {   // offsets into the workspace in floats (each region 128-byte aligned); total * 4 bytes in all
+struct DetBwdWs {  // [weight slots | segment slots | rot], each 128-byte aligned, rot padded to 256 bytes
   int grid_max;
-  size_t seg, rot, total;   // rot: grad_R of every item [B*N][9] for a shared R (its sum over pairs)
-  DetBwdWs(int B, int64_t N, bool shared_grad_R)
+  float *w, *seg, *rot;  // rot: grad_R of every item [B*N][9] for a shared R (its sum over pairs)
+  DetBwdWs(Carve& c, int B, int64_t N, bool shared_grad_R)
       : grid_max((int)((int64_t)B * N < kDetGridCap ? (int64_t)B * N : kDetGridCap)),
-        seg((size_t)grid_max * kDetWSlot),
-        rot(seg + (B > 0 && grid_max > 0 ? (size_t)(grid_max + B - 1) * kDetSegSlot : 0)),
-        total(rot + (shared_grad_R ? ((size_t)B * (size_t)N * 9 + 63) / 64 * 64 : 0)) {}
+        w(c.take<float>((size_t)grid_max * kDetWSlot, 128)),
+        seg(c.take<float>(B > 0 && grid_max > 0 ? (size_t)(grid_max + B - 1) * kDetSegSlot : 0, 128)),
+        rot(c.take<float>(shared_grad_R ? (size_t)B * (size_t)N * 9 : 0, 256)) {}
 };
-int launch_score_bwd_det(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
-                         const float* W1, const float* W2, const float* b2, const float* base, const float* grad_scores,
-                         const void* h1_saved, const float* pair_inv, float* g_vol, float* g_tgt, float* g_W1,
-                         float* g_W2, float* g_b2, float* g_R, int B, int64_t N, bool tc, float* ws, cudaStream_t s);
-int launch_score_tc_train(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair, const float* W1,
-                          const float* W2, const float* b2, const float* base, float* scores, void* h1_out,
-                          float* pair_inv_out, int B, int64_t N, void* ws, size_t ws_bytes, cudaStream_t s);
+int launch_score_bwd_det(const Scored& p, const float* tgt_feat, const float* grad_scores, const void* h1_saved,
+                         const float* pair_inv, float* g_vol, float* g_tgt, float* g_W1, float* g_W2, float* g_b2,
+                         float* g_R, bool tc, const DetBwdWs& w, cudaStream_t s);
 int launch_resblock3d(const float* x, const float* Wc1, const float* Wc2, const float* Wd, float* out, int64_t m,
                       cudaStream_t s);
 int launch_infonce(const float* scores, const float* R, int r_per_pair, const float* gt, float thr_deg, float temperature,
                    float* loss, float* grad, int B, int64_t N, cudaStream_t s);
-int launch_gradient_ascent(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R_init, const float* W1,
-                           const float* W2, const float* b2, const float* base, int steps, float step_deg, float* R_out,
-                           float* score_out, int B, int K, cudaStream_t s, const int64_t* skip_idx = nullptr,
-                           int64_t item_lo = 0, int64_t item_hi = -1);  // item_hi < 0: every item of B*K
+// p: the starting rotations R_init [B][K][9] (per pair, N = K)
+int launch_gradient_ascent(const Scored& p, const float* tgt_feat, int steps, float step_deg, float* R_out,
+                           float* score_out, cudaStream_t s, const int64_t* skip_idx = nullptr, int64_t item_lo = 0,
+                           int64_t item_hi = -1);  // item_hi < 0: every item of B*K
 int launch_forward_3d2d(const float* vol, const float* W1, const float* W2, const float* b2,
                         float* feat, int64_t m, cudaStream_t s);
 int launch_tgt_feat(const float* vol_tgt, const float* W1, const float* W2, const float* b2,
                     unsigned long long* clear_keys, float* feat, int B, cudaStream_t s);
-int launch_score_fp32(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R,
-                      int r_per_pair, const float* W1, const float* W2, const float* b2,
-                      const float* base, float* scores, int B, int64_t N, cudaStream_t s);
-int launch_score_tc(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R,
-                    int r_per_pair, const float* W1, const float* W2, const float* b2,
-                    const float* base, float* scores, int B, int64_t N, void* ws, size_t ws_bytes,
-                    cudaStream_t s, bool f16_gather);
-size_t score_tc_workspace_bytes(int B, int64_t N);
-float* scratch_tgt_feat(void* ws, int B);  // [B,32,64] slot inside the tensor-core scratch
-int launch_verify_tc_argmax(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R,
-                            int r_per_pair, const float* W1, const float* W2, const float* b2,
-                            const float* base, float* scores, float* best_val, int64_t* best_idx,
-                            float* R_best, int64_t idx_offset, int B, int64_t N, void* ws, size_t ws_bytes,
-                            cudaStream_t s, bool f16_gather, const peer::Args* pa = nullptr);
-int launch_verify_tc_screened(const float* vol_src, const float* vol_tgt, const float* R, int r_per_pair, const float* W1,
-                              const float* W2, const float* b2, const float* base, float* best_val, int64_t* best_idx,
-                              float* R_best, int64_t idx_offset, int B, int64_t N, void* ws, size_t ws_bytes, float* s16,
-                              void* lists, cudaStream_t s, const peer::Args* pa = nullptr);
+int launch_score_fp32(const Scored& p, const float* tgt_feat, float* scores, cudaStream_t s);
+// The tensor-core scorers' scratch, packed.  The reserved regions keep the workspace sizes, which callers see, as they
+// are.  launch_tgt_feat clears the keys and the counter that follows them together.
+struct TcScratch {
+  float* tgt_feat;                // [B,32,64]
+  unsigned long long* best_keys;  // [B] arg-max keys
+  unsigned* counter;              // first word of a 256-byte tail
+  TcScratch() = default;
+  TcScratch(Carve& c, int B) {
+    c.take<unsigned char>(26 * 1024, 1);  // reserved
+    tgt_feat = c.take<float>((size_t)B * kO * kP, 1);
+    c.take<float2>(B, 1);  // reserved
+    best_keys = c.take<unsigned long long>(B, 1);
+    counter = c.take<unsigned>(64, 1);
+  }
+};
+int launch_score_tc(const Scored& p, const float* tgt_feat, float* scores, const TcScratch& sc, cudaStream_t s,
+                    bool f16_gather);
+int launch_score_tc_train(const Scored& p, const float* tgt_feat, float* scores, void* h1_out, float* pair_inv_out,
+                          const TcScratch& sc, cudaStream_t s);
+// Screened arg-max of ahv_verify (k = 1, fp32 volumes, AHV_MATH_TC; the passes are described at
+// launch_verify_tc_screened in ahv_score_tc.cu).  Per pair a list of kScreenList hypotheses: the contenders (16-bit
+// gather score within 2 tau of the pair's screened maximum, at most kScreenCap of them, padded with the first), then
+// kScreenProbes fixed strided probes.  tau is in score units (scores are means of cosines): 27x the largest 16-bit vs
+// fp32 gather difference on the bench workload (7.3e-5) and at least 8x that of order-one volumes with outliers up to
+// 3e7 times the bulk, of the mixed per-pair scales and of the head-weight cases short of one W1 row dominating the
+// others by 2^6 (profiles/r11_screen_margin.json); with it the bench workload has at most 22 contenders per pair.
+constexpr int kScreenCap = 224;
+constexpr int kScreenProbes = 32;
+constexpr int kScreenList = kScreenCap + kScreenProbes;
+constexpr float kScreenTau = 2e-3f;
+struct ScreenLists {  // packed, in this order; passed by value to the kernels
+  int* idx;      // [B][kScreenList] hypothesis index
+  float* s16;    // [B][kScreenList] its 16-bit gather score
+  int* count;    // [B] contenders found (more than kScreenCap: the pair is flagged)
+  float* err;    // [B] largest |fp32 score - 16-bit score| over the list
+  int* flagged;  // [1 + B]: number of flagged pairs, then the flagged pairs (in no particular order)
+  ScreenLists() = default;
+  ScreenLists(Carve& c, int B)
+      : idx(c.take<int>((size_t)B * kScreenList, 1)),
+        s16(c.take<float>((size_t)B * kScreenList, 1)),
+        count(c.take<int>(B, 1)),
+        err(c.take<float>(B, 1)),
+        flagged(c.take<int>((size_t)B + 1, 1)) {}
+};
+// the fused k = 1 verification with target features computed from vol_tgt
+int launch_verify_tc_argmax(const Scored& p, const float* vol_tgt, float* scores, float* best_val, int64_t* best_idx,
+                            float* R_best, int64_t idx_offset, const TcScratch& sc, cudaStream_t s, bool f16_gather,
+                            const peer::Args* pa);
+int launch_verify_tc_screened(const Scored& p, const float* vol_tgt, float* best_val, int64_t* best_idx, float* R_best,
+                              int64_t idx_offset, const TcScratch& sc, float* s16, const ScreenLists& L, cudaStream_t s,
+                              const peer::Args* pa);
 int launch_topk_exchange(const float* val, const int64_t* idx, const float* R, int r_per_pair, int64_t idx_offset,
                          int64_t N, int B, int k, float* out_val, int64_t* out_idx, float* R_best,
                          const peer::Args& pa, cudaStream_t s);
@@ -244,37 +311,11 @@ int launch_modes_beams(const float* S0, const float* G, int64_t n0, const int64_
                        int k, int w, float min_sep_deg, uint8_t* slot, int64_t* par, int64_t* gen, cudaStream_t s);
 int launch_modes_level(const float* sc, const int64_t* kids, const float* kids_R, int B, int k, int w, bool last,
                        int64_t* par, int64_t* gen, float* val, int64_t* idx, float* R_out, cudaStream_t s);
-// Screened arg-max of ahv_verify (k = 1, fp32 volumes, AHV_MATH_TC; the passes are described at
-// launch_verify_tc_screened in ahv_score_tc.cu).  Per pair a list of kScreenList hypotheses: the contenders (16-bit
-// gather score within 2 tau of the pair's screened maximum, at most kScreenCap of them, padded with the first), then
-// kScreenProbes fixed strided probes.  tau is in score units (scores are means of cosines): 27x the largest 16-bit vs
-// fp32 gather difference on the bench workload (7.3e-5) and at least 8x that of order-one volumes with outliers up to
-// 3e7 times the bulk, of the mixed per-pair scales and of the head-weight cases short of one W1 row dominating the
-// others by 2^6 (profiles/r11_screen_margin.json); with it the bench workload has at most 22 contenders per pair.
-constexpr int kScreenCap = 224;
-constexpr int kScreenProbes = 32;
-constexpr int kScreenList = kScreenCap + kScreenProbes;
-constexpr float kScreenTau = 2e-3f;
-struct ScreenLists {  // carved from the verification workspace's top-k partials region (unused when k == 1)
-  int* idx;      // [B][kScreenList] hypothesis index
-  float* s16;    // [B][kScreenList] its 16-bit gather score
-  int* count;    // [B] contenders found (more than kScreenCap: the pair is flagged)
-  float* err;    // [B] largest |fp32 score - 16-bit score| over the list
-  int* flagged;  // [1 + B]: number of flagged pairs, then the flagged pairs (in no particular order)
-  static size_t bytes(int B) { return (size_t)B * kScreenList * 8 + (size_t)B * 8 + (size_t)(B + 1) * 4; }
-  ScreenLists(void* p, int B) {
-    idx = static_cast<int*>(p);
-    s16 = reinterpret_cast<float*>(idx + (size_t)B * kScreenList);
-    count = reinterpret_cast<int*>(s16 + (size_t)B * kScreenList);
-    err = reinterpret_cast<float*>(count + B);
-    flagged = reinterpret_cast<int*>(err + B);
-  }
-};
 int launch_screen_select(const float* s16, const unsigned long long* keys, int B, int64_t N, const float* R, int r_per_pair,
                          const ScreenLists& L, float* R_list, cudaStream_t s);
 int launch_screen_guard(const float* s32, const ScreenLists& L, int B, unsigned long long* keys, cudaStream_t s);
-size_t posterior_workspace_bytes(int B, int64_t N, int k, bool moments);
 // ahv_posterior_mass (moment == nullptr) and ahv_posterior_moments (mean_R, mean_cos and moment set)
+size_t posterior_workspace_bytes(int B, int64_t N, int k, bool moments);
 int launch_posterior(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N, int k,
                      float radius_deg, float temperature, float* log_z, float* mass, float* mean_R, float* mean_cos,
                      float* moment, void* ws, cudaStream_t s);

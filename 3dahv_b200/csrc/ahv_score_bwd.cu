@@ -278,12 +278,10 @@ score_bwd_kernel(const float* __restrict__ vol_src, const float* __restrict__ tg
   }
 }
 
-int launch_score_bwd(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
-                     const float* W1, const float* W2, const float* b2, const float* base,
-                     const float* grad_scores, float* g_vol, float* g_tgt, float* g_W1, float* g_W2,
-                     float* g_b2, int B, int64_t N, cudaStream_t s, const void* h1_saved, const float* pair_inv,
+int launch_score_bwd(const Scored& p, const float* tgt_feat, const float* grad_scores, float* g_vol, float* g_tgt,
+                     float* g_W1, float* g_W2, float* g_b2, cudaStream_t s, const void* h1_saved, const float* pair_inv,
                      float* g_R, unsigned grid, bool det) {
-  const int64_t total = (int64_t)B * N;
+  const int64_t total = (int64_t)p.B * p.N;
   if (total == 0) return AHV_OK;
   if (grid == 0) {
     const int sms = sm_count();
@@ -295,8 +293,9 @@ int launch_score_bwd(const float* vol_src, const float* tgt_feat, const float* R
                          : (det ? score_bwd_kernel<false, true> : score_bwd_kernel<false, false>);
   const size_t smem = sizeof(BwdSmem);
   AHV_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kernel<<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores, g_vol, g_tgt,
-                                      g_W1, g_W2, g_b2, B, N, static_cast<const __half*>(h1_saved), pair_inv, g_R);
+  kernel<<<grid, kThreads, smem, s>>>(p.vol_f32(), tgt_feat, p.R, p.r_per_pair, p.W1, p.W2, p.b2, p.base, grad_scores,
+                                      g_vol, g_tgt, g_W1, g_W2, g_b2, p.B, p.N, static_cast<const __half*>(h1_saved),
+                                      pair_inv, g_R);
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }
@@ -350,33 +349,32 @@ score_bwd_det_reduce(const float* __restrict__ ws, size_t seg_off, size_t rot_of
   }
 }
 
-int launch_score_bwd_det(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
-                         const float* W1, const float* W2, const float* b2, const float* base, const float* grad_scores,
-                         const void* h1_saved, const float* pair_inv, float* g_vol, float* g_tgt, float* g_W1,
-                         float* g_W2, float* g_b2, float* g_R, int B, int64_t N, bool tc, float* ws, cudaStream_t s) {
-  const int64_t total = (int64_t)B * N;
+int launch_score_bwd_det(const Scored& p, const float* tgt_feat, const float* grad_scores, const void* h1_saved,
+                         const float* pair_inv, float* g_vol, float* g_tgt, float* g_W1, float* g_W2, float* g_b2,
+                         float* g_R, bool tc, const DetBwdWs& w, cudaStream_t s) {
+  const int B = p.B;
+  const int64_t N = p.N, total = (int64_t)B * N;
   if (total == 0) return AHV_OK;
   const int sms = sm_count();
   if (sms <= 0) return AHV_ECUDA;
   const int grid = (int)std::min<int64_t>(total, std::min(sms, kDetGridCap));
-  const bool shared_R = g_R && !r_per_pair;
-  const DetBwdWs w(B, N, shared_R);
+  const bool shared_R = g_R && !p.r_per_pair;
   // the kernel's outputs are the workspace slots (NULL where the caller's output is NULL); a per-pair R's gradient
   // has one writer per element and goes straight to the caller's buffer
-  float* k_vol = g_vol ? ws + w.seg : nullptr;
-  float* k_tgt = g_tgt ? ws + w.seg + kC * kVox : nullptr;
-  float* k_W1 = g_W1 ? ws : nullptr;
-  float* k_W2 = g_W2 ? ws + kO * kK : nullptr;
-  float* k_b2 = g_b2 ? ws + kO * kK + kO * kO : nullptr;
-  float* k_R = g_R ? (r_per_pair ? g_R : ws + w.rot) : nullptr;
-  const int st = tc ? launch_score_bwd_tc(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores, h1_saved,
-                                          pair_inv, k_vol, k_tgt, k_W1, k_W2, k_b2, B, N, s, (unsigned)grid, true)
-                    : launch_score_bwd(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores, k_vol, k_tgt,
-                                       k_W1, k_W2, k_b2, B, N, s, h1_saved, pair_inv, k_R, (unsigned)grid, true);
+  float* k_vol = g_vol ? w.seg : nullptr;
+  float* k_tgt = g_tgt ? w.seg + kC * kVox : nullptr;
+  float* k_W1 = g_W1 ? w.w : nullptr;
+  float* k_W2 = g_W2 ? w.w + kO * kK : nullptr;
+  float* k_b2 = g_b2 ? w.w + kO * kK + kO * kO : nullptr;
+  float* k_R = g_R ? (p.r_per_pair ? g_R : w.rot) : nullptr;
+  const int st = tc ? launch_score_bwd_tc(p, tgt_feat, grad_scores, h1_saved, pair_inv, k_vol, k_tgt, k_W1, k_W2, k_b2, s,
+                                          (unsigned)grid, true)
+                    : launch_score_bwd(p, tgt_feat, grad_scores, k_vol, k_tgt, k_W1, k_W2, k_b2, s, h1_saved, pair_inv, k_R,
+                                       (unsigned)grid, true);
   if (st != AHV_OK) return st;
   const int64_t n_all = kDetWSlot + (int64_t)B * kDetSegSlot + (shared_R ? N * 9 : 0);
   const unsigned blocks = (unsigned)std::min<int64_t>((n_all + 255) / 256, 8 * (int64_t)sms);
-  score_bwd_det_reduce<<<blocks, 256, 0, s>>>(ws, w.seg, w.rot, grid, B, N, g_vol, g_tgt, g_W1, g_W2, g_b2,
+  score_bwd_det_reduce<<<blocks, 256, 0, s>>>(w.w, w.seg - w.w, w.rot - w.w, grid, B, N, g_vol, g_tgt, g_W1, g_W2, g_b2,
                                               shared_R ? g_R : nullptr);
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;

@@ -759,12 +759,10 @@ score_bwd_tc_kernel(const float* __restrict__ vol_src, const float* __restrict__
 
 }  // namespace
 
-int launch_score_bwd_tc(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair,
-                        const float* W1, const float* W2, const float* b2, const float* base,
-                        const float* grad_scores, const void* h1_saved, const float* pair_inv, float* g_vol,
-                        float* g_tgt, float* g_W1, float* g_W2, float* g_b2, int B, int64_t N, cudaStream_t s,
-                        unsigned grid, bool det) {
-  const int64_t total = (int64_t)B * N;
+int launch_score_bwd_tc(const Scored& p, const float* tgt_feat, const float* grad_scores, const void* h1_saved,
+                        const float* pair_inv, float* g_vol, float* g_tgt, float* g_W1, float* g_W2, float* g_b2,
+                        cudaStream_t s, unsigned grid, bool det) {
+  const int64_t total = (int64_t)p.B * p.N;
   if (total == 0) return AHV_OK;
   if (!h1_saved || !pair_inv) return AHV_EINVAL;
   if (grid == 0) {
@@ -775,8 +773,9 @@ int launch_score_bwd_tc(const float* vol_src, const float* tgt_feat, const float
   const auto kernel = det ? score_bwd_tc_kernel<true> : score_bwd_tc_kernel<false>;
   const size_t smem = sizeof(BwdTcSmem);
   AHV_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kernel<<<grid, kThreads, smem, s>>>(vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, grad_scores,
-                                      static_cast<const __half*>(h1_saved), pair_inv, g_vol, g_tgt, g_W1, g_W2, g_b2, B, N);
+  kernel<<<grid, kThreads, smem, s>>>(p.vol_f32(), tgt_feat, p.R, p.r_per_pair, p.W1, p.W2, p.b2, p.base, grad_scores,
+                                      static_cast<const __half*>(h1_saved), pair_inv, g_vol, g_tgt, g_W1, g_W2, g_b2, p.B,
+                                      p.N);
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;
 }

@@ -264,25 +264,23 @@ int launch_rotate_volume_grad_R(const float* vol, int per_rot, const float* R, c
 
 // ---- launchers --------------------------------------------------------------
 
-int launch_score_fp32(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R,
-                      int r_per_pair, const float* W1, const float* W2, const float* b2,
-                      const float* base, float* scores, int B, int64_t N, cudaStream_t s) {
-  const int64_t total = (int64_t)B * N;
+int launch_score_fp32(const Scored& p, const float* tgt_feat, float* scores, cudaStream_t s) {
+  const int64_t total = (int64_t)p.B * p.N;
   if (total == 0) return AHV_OK;
   const int sms = sm_count();
   if (sms <= 0) return AHV_ECUDA;
   const unsigned grid = (unsigned)(total < sms ? total : sms);
   const size_t smem = sizeof(Fp32Smem);
-  if (vol_dtype == AHV_VOL_F32) {
+  if (p.vol_dtype == AHV_VOL_F32) {
     AHV_CUDA_OK(cudaFuncSetAttribute(score_fp32_kernel<float>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    score_fp32_kernel<float><<<grid, kThreads, smem, s>>>((const float*)vol_src, tgt_feat, R,
-                                                          r_per_pair, W1, W2, b2, base, scores, B, N);
+    score_fp32_kernel<float><<<grid, kThreads, smem, s>>>(p.vol_f32(), tgt_feat, p.R, p.r_per_pair, p.W1, p.W2, p.b2,
+                                                          p.base, scores, p.B, p.N);
   } else {
     AHV_CUDA_OK(cudaFuncSetAttribute(score_fp32_kernel<__nv_bfloat16>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     score_fp32_kernel<__nv_bfloat16><<<grid, kThreads, smem, s>>>(
-        (const __nv_bfloat16*)vol_src, tgt_feat, R, r_per_pair, W1, W2, b2, base, scores, B, N);
+        (const __nv_bfloat16*)p.vol_src, tgt_feat, p.R, p.r_per_pair, p.W1, p.W2, p.b2, p.base, scores, p.B, p.N);
   }
   AHV_CUDA_OK(cudaGetLastError());
   return AHV_OK;

@@ -42,7 +42,7 @@
 //
 // Files: ahv_tc_ptx.cuh (PTX wrappers), ahv_peer.cuh (NVLink exchange buffer), ahv_tc_common.cuh (roles, tile
 // iterator, weight packing, volume staging, epilogue), ahv_score_tc_ts.cuh (the kernel), this file
-// (target-feature prologue, workspace carve-up, launchers).
+// (target-feature prologue, launchers).
 #include "ahv_score_tc_ts.cuh"
 
 namespace ahv {
@@ -123,30 +123,6 @@ tc_tgt_feat_kernel(const float* __restrict__ vol_tgt, const float* __restrict__ 
   }
 }
 
-struct Scratch {  // carve-up of the tensor-core path's workspace
-  __half* w_packed;
-  float2* pair_scale;
-  u64* best_keys;
-  unsigned* counter;
-  float* tgt_feat;
-};
-__host__ inline size_t scratch_bytes(int B) {
-  return (size_t)(kW1Bytes + kW2Bytes) + (size_t)B * (sizeof(float2) + sizeof(u64)) + (size_t)B * kO * kP * 4 + 256;
-}
-__host__ inline Scratch carve(void* ws, int B) {
-  unsigned char* p = static_cast<unsigned char*>(ws);
-  Scratch sc;
-  sc.w_packed = reinterpret_cast<__half*>(p);
-  p += kW1Bytes + kW2Bytes;
-  sc.tgt_feat = reinterpret_cast<float*>(p);
-  p += (size_t)B * kO * kP * 4;
-  sc.pair_scale = reinterpret_cast<float2*>(p);
-  p += (size_t)B * sizeof(float2);
-  sc.best_keys = reinterpret_cast<u64*>(p);
-  sc.counter = reinterpret_cast<unsigned*>(sc.best_keys + B);  // inside the 256-byte tail of scratch_bytes
-  return sc;
-}
-
 // Tensor map of the source volumes for the TMA staging: [B*16 channels][8 d][64 (h,w)] elements, one box = one
 // pair's whole volume (contiguous in HBM; the 3-D form keeps every box dimension <= 256).
 static int make_volume_map(const void* vol_src, int B, bool bf16, CUtensorMap* map) {
@@ -196,16 +172,16 @@ static int launch_pdl(KernelT kernel, unsigned grid, size_t smem, cudaStream_t s
 // dependent on it (its setup, weight packing, volume staging and first gathers overlap the prologue; only
 // the epilogue warps wait for the target features).
 template <typename T, bool K16, bool kSave = false>
-int launch_typed(const T* vol_src, const float* vol_tgt, const float* tgt_feat_in, const float* R,
-                 int r_per_pair, const float* W1, const float* W2, const float* b2, const float* base,
-                 float* scores, bool want_argmax, int B, int64_t N, const Scratch& sc, Finalize fin, cudaStream_t s,
-                 const int* pair_list = nullptr) {
+int launch_typed(const Scored& p, const float* vol_tgt, const float* tgt_feat_in, float* scores, bool want_argmax,
+                 const TcScratch& sc, Finalize fin, cudaStream_t s, const int* pair_list = nullptr) {
+  const int B = p.B;
+  const int64_t N = p.N;
   int dev = 0, sms = 0;
   AHV_CUDA_OK(cudaGetDevice(&dev));
   AHV_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   const bool prologue = vol_tgt != nullptr;
   if (prologue) {
-    const int st = launch_tgt_feat(vol_tgt, W1, W2, b2, want_argmax ? sc.best_keys : nullptr, sc.tgt_feat, B, s);
+    const int st = launch_tgt_feat(vol_tgt, p.W1, p.W2, p.b2, want_argmax ? sc.best_keys : nullptr, sc.tgt_feat, B, s);
     if (st != AHV_OK) return st;
   } else if (want_argmax && !pair_list) {  // a listed-pairs pass adds to the keys (and the cleared counter) it finds
     AHV_CUDA_OK(cudaMemsetAsync(sc.best_keys, 0, (size_t)B * sizeof(u64) + sizeof(unsigned), s));
@@ -218,15 +194,15 @@ int launch_typed(const T* vol_src, const float* vol_tgt, const float* tgt_feat_i
   const float* tgt = prologue ? sc.tgt_feat : tgt_feat_in;
   u64* keys = want_argmax ? sc.best_keys : nullptr;
   CUtensorMap vol_map;
-  const int mst = make_volume_map(vol_src, B, sizeof(T) == 2, &vol_map);
+  const int mst = make_volume_map(p.vol_src, B, sizeof(T) == 2, &vol_map);
   if (mst != AHV_OK) return mst;
   AHV_CUDA_OK(cudaFuncSetAttribute(score_tc_ts_kernel<T, K16, kSave>, cudaFuncAttributeMaxDynamicSharedMemorySize, MapTS::smem_bytes));
   // CTAs that inherit the prologue's SMs start late; only worth compensating when the prologue is smaller than this
   // grid and every CTA has tiles to spare (see the work split in the kernel)
   int late = 0;
   if (prologue && kTgtCtasPerPair * (int64_t)B <= grid / 2 && (int64_t)B * N / grid >= 8) late = kTgtCtasPerPair * B;
-  return launch_pdl(score_tc_ts_kernel<T, K16, kSave>, grid, MapTS::smem_bytes, s, prologue, vol_map, tgt, R, r_per_pair, b2, base, W1,
-                    W2, scores, keys, B, N, fin, late, pair_list);
+  return launch_pdl(score_tc_ts_kernel<T, K16, kSave>, grid, MapTS::smem_bytes, s, prologue, vol_map, tgt, p.R,
+                    (int)p.r_per_pair, p.b2, p.base, p.W1, p.W2, scores, keys, B, N, fin, late, pair_list);
 }
 
 }  // namespace tc
@@ -243,59 +219,38 @@ int launch_tgt_feat(const float* vol_tgt, const float* W1, const float* W2, cons
     const int nb = B - b0 < 65535 ? B - b0 : 65535;
     tc::tc_tgt_feat_kernel<<<dim3(tc::kTgtCtasPerPair, nb), tc::kTgtThreads, 0, s>>>(
         vol_tgt + (size_t)b0 * kC * kVox, W1, W2, b2, clear_keys ? clear_keys + b0 : nullptr,
-        clear_keys && b0 == 0 ? reinterpret_cast<unsigned*>(clear_keys + B) : nullptr,  // Scratch::counter
+        clear_keys && b0 == 0 ? reinterpret_cast<unsigned*>(clear_keys + B) : nullptr,  // TcScratch::counter
         feat + (size_t)b0 * kO * kP, nb);
     AHV_CUDA_OK(cudaGetLastError());
   }
   return AHV_OK;
 }
 
-size_t score_tc_workspace_bytes(int B, int64_t N) {
-  (void)N;
-  return tc::scratch_bytes(B);
-}
-
-float* scratch_tgt_feat(void* ws, int B) { return tc::carve(ws, B).tgt_feat; }
-
 // dispatch on (volume dtype, gather precision): bf16 volumes always use the 16-bit staged gather
 // (exact staging); fp32 volumes use it only when the caller opts in (AHV_MATH_TC_F16GATHER)
-static int dispatch(const void* vol_src, int vol_dtype, bool f16_gather, const float* vol_tgt,
-                    const float* tgt_feat, const float* R, int r_per_pair, const float* W1, const float* W2,
-                    const float* b2, const float* base, float* scores, bool want_argmax, int B, int64_t N,
-                    const tc::Scratch& sc, const tc::Finalize& fin, cudaStream_t s) {
-  if (vol_dtype == AHV_VOL_BF16)
-    return tc::launch_typed<__nv_bfloat16, true>((const __nv_bfloat16*)vol_src, vol_tgt, tgt_feat, R, r_per_pair, W1,
-                                                 W2, b2, base, scores, want_argmax, B, N, sc, fin, s);
-  if (f16_gather)
-    return tc::launch_typed<float, true>((const float*)vol_src, vol_tgt, tgt_feat, R, r_per_pair, W1, W2, b2, base,
-                                         scores, want_argmax, B, N, sc, fin, s);
-  return tc::launch_typed<float, false>((const float*)vol_src, vol_tgt, tgt_feat, R, r_per_pair, W1, W2, b2, base,
-                                        scores, want_argmax, B, N, sc, fin, s);
+static int dispatch(const Scored& p, bool f16_gather, const float* vol_tgt, const float* tgt_feat, float* scores,
+                    bool want_argmax, const TcScratch& sc, const tc::Finalize& fin, cudaStream_t s) {
+  if (p.vol_dtype == AHV_VOL_BF16)
+    return tc::launch_typed<__nv_bfloat16, true>(p, vol_tgt, tgt_feat, scores, want_argmax, sc, fin, s);
+  if (f16_gather) return tc::launch_typed<float, true>(p, vol_tgt, tgt_feat, scores, want_argmax, sc, fin, s);
+  return tc::launch_typed<float, false>(p, vol_tgt, tgt_feat, scores, want_argmax, sc, fin, s);
 }
 
 // scores only (target features supplied by the caller)
-int launch_score_tc(const void* vol_src, int vol_dtype, const float* tgt_feat, const float* R,
-                    int r_per_pair, const float* W1, const float* W2, const float* b2,
-                    const float* base, float* scores, int B, int64_t N, void* ws, size_t ws_bytes,
-                    cudaStream_t s, bool f16_gather) {
-  if ((int64_t)B * N == 0) return AHV_OK;
-  if (ws_bytes < tc::scratch_bytes(B)) return AHV_EWORKSPACE;
-  return dispatch(vol_src, vol_dtype, f16_gather, nullptr, tgt_feat, R, r_per_pair, W1, W2, b2, base, scores, false,
-                  B, N, tc::carve(ws, B), tc::Finalize{}, s);
+int launch_score_tc(const Scored& p, const float* tgt_feat, float* scores, const TcScratch& sc, cudaStream_t s,
+                    bool f16_gather) {
+  if ((int64_t)p.B * p.N == 0) return AHV_OK;
+  return dispatch(p, f16_gather, nullptr, tgt_feat, scores, false, sc, tc::Finalize{}, s);
 }
 
 // training forward (modules/model.py:53-56 before autograd): scores + the ReLU'd conv1 output of every item and the
 // pair scales, which ahv_score_backward's saved-activation form reads instead of recomputing conv1
-int launch_score_tc_train(const float* vol_src, const float* tgt_feat, const float* R, int r_per_pair, const float* W1,
-                          const float* W2, const float* b2, const float* base, float* scores, void* h1_out,
-                          float* pair_inv_out, int B, int64_t N, void* ws, size_t ws_bytes, cudaStream_t s) {
-  if ((int64_t)B * N == 0) return AHV_OK;
-  if (ws_bytes < tc::scratch_bytes(B)) return AHV_EWORKSPACE;
+int launch_score_tc_train(const Scored& p, const float* tgt_feat, float* scores, void* h1_out, float* pair_inv_out,
+                          const TcScratch& sc, cudaStream_t s) {
   tc::Finalize fin;
   fin.h1_out = static_cast<__half*>(h1_out);
   fin.pair_inv_out = pair_inv_out;
-  return tc::launch_typed<float, false, true>(vol_src, nullptr, tgt_feat, R, r_per_pair, W1, W2, b2, base, scores, false, B, N,
-                                              tc::carve(ws, B), fin, s);
+  return tc::launch_typed<float, false, true>(p, nullptr, tgt_feat, scores, false, sc, fin, s);
 }
 
 // the fused selection of a k = 1 verification: winners decoded by the scoring kernel's last CTA, or exchanged with the
@@ -318,19 +273,15 @@ static int make_finalize(float* best_val, int64_t* best_idx, float* R_best, int6
 
 // the whole verification step with arg-max selection in two launches: prologue (target features, key
 // clear) -> fused scoring + arg-max, whose last CTA also decodes the winners (no finalize launch)
-int launch_verify_tc_argmax(const void* vol_src, int vol_dtype, const float* vol_tgt, const float* R,
-                            int r_per_pair, const float* W1, const float* W2, const float* b2,
-                            const float* base, float* scores, float* best_val, int64_t* best_idx,
-                            float* R_best, int64_t idx_offset, int B, int64_t N, void* ws, size_t ws_bytes,
-                            cudaStream_t s, bool f16_gather, const peer::Args* pa) {
+int launch_verify_tc_argmax(const Scored& p, const float* vol_tgt, float* scores, float* best_val, int64_t* best_idx,
+                            float* R_best, int64_t idx_offset, const TcScratch& sc, cudaStream_t s, bool f16_gather,
+                            const peer::Args* pa) {
   const int world = pa ? pa->world : 1;
-  if ((int64_t)B * N == 0) return world > 1 ? AHV_EINVAL : AHV_OK;  // a sharded step needs every rank in the exchange
-  if (ws_bytes < tc::scratch_bytes(B)) return AHV_EWORKSPACE;
+  if ((int64_t)p.B * p.N == 0) return world > 1 ? AHV_EINVAL : AHV_OK;  // a sharded step needs every rank in the exchange
   tc::Finalize fin;
-  const int st = make_finalize(best_val, best_idx, R_best, idx_offset, B, pa, &fin);
+  const int st = make_finalize(best_val, best_idx, R_best, idx_offset, p.B, pa, &fin);
   if (st != AHV_OK) return st;
-  return dispatch(vol_src, vol_dtype, f16_gather, vol_tgt, nullptr, R, r_per_pair, W1, W2, b2, base, scores, true,
-                  B, N, tc::carve(ws, B), fin, s);
+  return dispatch(p, f16_gather, vol_tgt, nullptr, scores, true, sc, fin, s);
 }
 
 // The same step for fp32 volumes with the fp32 gather's result, screened by the 16-bit gather (1.6x its rate):
@@ -346,32 +297,27 @@ int launch_verify_tc_argmax(const void* vol_src, int vol_dtype, const float* vol
 // A hypothesis's score depends on (pair, rotation) alone, not on the tile or CTA it is scored in, so the fp32 winner is
 // the single pass's bit for bit whenever it is on its pair's list - which holds when every 16-bit score lies within
 // tau of its fp32 score: then s16[w] >= s32[w] - tau >= s32[n*] - tau >= m_b - 2 tau (n* the screened arg-max).
-// `s16` must hold B*N floats and at least kScreenList*40 bytes per pair; `lists` ScreenLists::bytes(B).  No host
+// `s16` must hold B*N floats and at least kScreenList*40 bytes per pair.  No host
 // synchronisation: graph-capturable.
-int launch_verify_tc_screened(const float* vol_src, const float* vol_tgt, const float* R, int r_per_pair, const float* W1,
-                              const float* W2, const float* b2, const float* base, float* best_val, int64_t* best_idx,
-                              float* R_best, int64_t idx_offset, int B, int64_t N, void* ws, size_t ws_bytes, float* s16,
-                              void* lists, cudaStream_t s, const peer::Args* pa) {
-  if (ws_bytes < tc::scratch_bytes(B)) return AHV_EWORKSPACE;
+int launch_verify_tc_screened(const Scored& p, const float* vol_tgt, float* best_val, int64_t* best_idx, float* R_best,
+                              int64_t idx_offset, const TcScratch& sc, float* s16, const ScreenLists& L, cudaStream_t s,
+                              const peer::Args* pa) {
+  const int B = p.B;
   tc::Finalize fin;
   int st = make_finalize(best_val, best_idx, R_best, idx_offset, B, pa, &fin);
   if (st != AHV_OK) return st;
-  const tc::Scratch sc = tc::carve(ws, B);
-  const ScreenLists L(lists, B);
   float* R_list = s16;                                          // [B][kScreenList][9], after the selection
   float* s32 = s16 + (size_t)B * kScreenList * 9;               // [B][kScreenList]
-  st = tc::launch_typed<float, true>(vol_src, vol_tgt, nullptr, R, r_per_pair, W1, W2, b2, base, s16, true, B, N, sc,
-                                     tc::Finalize{}, s);
+  st = tc::launch_typed<float, true>(p, vol_tgt, nullptr, s16, true, sc, tc::Finalize{}, s);
   if (st != AHV_OK) return st;
-  st = launch_screen_select(s16, sc.best_keys, B, N, R, r_per_pair, L, R_list, s);
+  st = launch_screen_select(s16, sc.best_keys, B, p.N, p.R, p.r_per_pair, L, R_list, s);
   if (st != AHV_OK) return st;
-  st = tc::launch_typed<float, false>(vol_src, nullptr, sc.tgt_feat, R_list, 1, W1, W2, b2, base, s32, false, B, kScreenList,
-                                      sc, tc::Finalize{}, s);
+  st = tc::launch_typed<float, false>(p.with_R(R_list, true, kScreenList), nullptr, sc.tgt_feat, s32, false, sc,
+                                      tc::Finalize{}, s);
   if (st != AHV_OK) return st;
   st = launch_screen_guard(s32, L, B, sc.best_keys, s);
   if (st != AHV_OK) return st;
-  return tc::launch_typed<float, false>(vol_src, nullptr, sc.tgt_feat, R, r_per_pair, W1, W2, b2, base, nullptr, true, B, N,
-                                        sc, fin, s, L.flagged);
+  return tc::launch_typed<float, false>(p, nullptr, sc.tgt_feat, nullptr, true, sc, fin, s, L.flagged);
 }
 
 }  // namespace ahv

@@ -540,18 +540,24 @@ posterior_final_kernel(const double* __restrict__ ws_sum, const float* __restric
     final_moments(ws_mom + (size_t)b * chunks * k * 9, mc, chunks, k, T, m, live, bad, s_red, mean_R, mean_cos, moment);
 }
 
-struct Ws {
+struct Ws {  // [sums | maxima | moment records (moments)], each 256-byte aligned
   int chunks;
-  size_t max, mom, total;  // byte offsets: the sums at 0, the maxima at `max`, the moment records (kMoments) at `mom`
-  Ws(int B, int64_t N, int k, bool moments)
+  double* sum;
+  float* max;
+  double* mom;
+  Ws(Carve& c, int B, int64_t N, int k, bool moments)
       : chunks((int)((N + kChunk - 1) / kChunk)),
-        max(((size_t)B * chunks * (k + 1) * sizeof(double) + 255) / 256 * 256),
-        mom(max + ((size_t)B * chunks * sizeof(float) + 255) / 256 * 256),
-        total(mom + (moments ? ((size_t)B * chunks * k * 9 * sizeof(double) + 255) / 256 * 256 : 0)) {}
+        sum(c.take<double>((size_t)B * chunks * (k + 1), 256)),
+        max(c.take<float>((size_t)B * chunks, 256)),
+        mom(c.take<double>(moments ? (size_t)B * chunks * k * 9 : 0, 256)) {}
 };
 }  // namespace posterior
 
-size_t posterior_workspace_bytes(int B, int64_t N, int k, bool moments) { return posterior::Ws(B, N, k, moments).total; }
+size_t posterior_workspace_bytes(int B, int64_t N, int k, bool moments) {
+  Carve c;
+  (void)posterior::Ws(c, B, N, k, moments);
+  return c.off;
+}
 
 int launch_posterior(const float* scores, const float* R, int r_per_pair, const float* centers, int B, int64_t N, int k,
                      float radius_deg, float temperature, float* log_z, float* mass, float* mean_R, float* mean_cos,
@@ -559,26 +565,24 @@ int launch_posterior(const float* scores, const float* R, int r_per_pair, const 
   using namespace posterior;
   if (B == 0) return AHV_OK;
   const bool moments = moment != nullptr;
-  const Ws w(B, N, k, moments);
-  double* ws_sum = static_cast<double*>(ws);
-  float* ws_max = reinterpret_cast<float*>(static_cast<unsigned char*>(ws) + w.max);
-  double* ws_mom = moments ? reinterpret_cast<double*>(static_cast<unsigned char*>(ws) + w.mom) : nullptr;
+  Carve cur(ws);
+  const Ws w(cur, B, N, k, moments);
   const dim3 grid1((unsigned)w.chunks, (unsigned)(B < 65535 ? B : 65535));
   const float c = distinct::trace_threshold(radius_deg);
   const double T = (double)temperature;
   if (moments) {
-    posterior_chunk_kernel<true><<<grid1, kThreads, 0, s>>>(scores, R, r_per_pair, centers, B, N, k, c, T, w.chunks, ws_sum,
-                                                            ws_max, ws_mom);
+    posterior_chunk_kernel<true><<<grid1, kThreads, 0, s>>>(scores, R, r_per_pair, centers, B, N, k, c, T, w.chunks, w.sum,
+                                                            w.max, w.mom);
   } else {
     posterior_chunk_kernel<false><<<grid1, kThreads, 0, s>>>(scores, R, r_per_pair, centers, B, N, k, c, T, w.chunks,
-                                                             ws_sum, ws_max, nullptr);
+                                                             w.sum, w.max, nullptr);
   }
   AHV_CUDA_OK(cudaGetLastError());
   if (moments) {
-    posterior_final_kernel<true><<<(unsigned)B, kFinalThreads, 0, s>>>(ws_sum, ws_max, w.chunks, k, T, log_z, mass, ws_mom,
+    posterior_final_kernel<true><<<(unsigned)B, kFinalThreads, 0, s>>>(w.sum, w.max, w.chunks, k, T, log_z, mass, w.mom,
                                                                        mean_R, mean_cos, moment);
   } else {
-    posterior_final_kernel<false><<<(unsigned)B, kFinalThreads, 0, s>>>(ws_sum, ws_max, w.chunks, k, T, log_z, mass,
+    posterior_final_kernel<false><<<(unsigned)B, kFinalThreads, 0, s>>>(w.sum, w.max, w.chunks, k, T, log_z, mass,
                                                                         nullptr, nullptr, nullptr, nullptr);
   }
   AHV_CUDA_OK(cudaGetLastError());
