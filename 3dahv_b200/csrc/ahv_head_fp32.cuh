@@ -1,6 +1,6 @@
 // fp32 CUDA-core building blocks of the verification head (modules/modules.py:112-124),
-// shared by the AHV_MATH_FP32 scorer, ahv_forward_3d2d and the tensor-core path's prologue
-// (target features).  Shared-memory layout: see ahv_score_fp32.cu.
+// shared by the AHV_MATH_FP32 scorer, the gradient ascent and the backward kernels.  Shared-memory
+// layout: see ahv_score_fp32.cu.
 #pragma once
 #include "ahv_common.cuh"
 
@@ -56,18 +56,6 @@ __device__ __forceinline__ void stage_volume(float* __restrict__ vol, const T* _
     int z = v >> 6, y = (v >> 3) & 7, x = v & 7;
     int line = ((z + 1) * kHalo + (y + 1)) * kHalo + (x + 1);
     vol[line * kC + c] = to_f32<T>(vol_g[i]);
-  }
-}
-
-// plain (un-rotated) volume [16][512] -> rotA / rotT (forward_3d2d on its own)
-template <typename T>
-__device__ __forceinline__ void load_plain_volume(Fp32Smem& sm, const T* __restrict__ vol_g) {
-  for (int i = threadIdx.x; i < kC * kVox; i += kThreads) {
-    int c = i >> 9, v = i & 511;
-    int d = v >> 6, h = (v >> 3) & 7, w = v & 7;
-    float x = to_f32<T>(vol_g[i]);
-    sm.rotA[c * kRotC + d * kRotD + h * 8 + w] = x;
-    sm.rotT[c * kRotC + d * kRotD + w * 8 + h] = x;
   }
 }
 
@@ -257,29 +245,6 @@ __device__ __forceinline__ void mean_cosine(float ss, float dt, float* red, floa
     for (int w = 0; w < 8; ++w) tot += red[w];
     *out = tot * (1.0f / 64.0f);
   }
-}
-
-
-// One volume -> normalised features [32][64] (feat[o*64 + pos]); all 256 threads of the CTA.
-// Caller has staged the weights (stage_weights) and synchronised.
-template <typename T>
-__device__ __forceinline__ void forward_3d2d_block(Fp32Smem& sm, const T* __restrict__ vol_g,
-                                                   const float* b2r, float* __restrict__ feat_out) {
-  const int pos = threadIdx.x >> 2, cg2 = threadIdx.x & 3;
-  __syncthreads();
-  load_plain_volume<T>(sm, vol_g);
-  __syncthreads();
-  conv1_relu(sm);
-  __syncthreads();
-  float v[8];
-  conv2_bias(sm, b2r, v);
-  float ss = 0.0f;
-#pragma unroll
-  for (int oo = 0; oo < 8; ++oo) ss = fmaf(v[oo], v[oo], ss);
-  ss = quad_sum(ss);
-  const float inv = 1.0f / fmaxf(sqrtf(ss), 1e-12f);  // F.normalize eps (modules/modules.py:122)
-#pragma unroll
-  for (int oo = 0; oo < 8; ++oo) feat_out[(cg2 * 8 + oo) * kP + pos] = v[oo] * inv;
 }
 
 }  // namespace ahv

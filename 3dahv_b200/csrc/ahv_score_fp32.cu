@@ -4,8 +4,6 @@
 //    hypothesis) trilinear resample (utils.py:113-131) -> tri-plane head
 //    (modules/modules.py:112-124) -> cosine vs target -> mean.  Nothing is
 //    materialised in HBM except the 4-byte score.
-//  * forward_3d2d_kernel — modules/modules.py:112-124 on plain volumes
-//    (target features, refcompat).
 //  * rotate_volume_kernel — utils.py:113-131 materialised (refcompat only).
 //  * rotate_volume_bwd_kernel / rotate_volume_grad_R_kernel — its gradients w.r.t. the volume and the
 //    rotation (training variant, refcompat under autograd).
@@ -65,22 +63,6 @@ score_fp32_kernel(const T* __restrict__ vol_src, const float* __restrict__ tgt_f
     head_dots(v, tg, ss, dt);
     mean_cosine(ss, dt, sm.red, scores + it);
   }
-}
-
-// ---- forward_3d2d on plain volumes ----------------------------------------
-__global__ void __launch_bounds__(kThreads, 1)
-forward_3d2d_kernel(const float* __restrict__ vol, const float* __restrict__ W1,
-                    const float* __restrict__ W2, const float* __restrict__ b2,
-                    float* __restrict__ feat, int64_t M) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  Fp32Smem& sm = *reinterpret_cast<Fp32Smem*>(smem_raw);
-  stage_weights(sm, W1, W2, nullptr);
-  const int cg2 = threadIdx.x & 3;
-  float b2r[8];
-#pragma unroll
-  for (int oo = 0; oo < 8; ++oo) b2r[oo] = b2[cg2 * 8 + oo];
-  for (int64_t m = blockIdx.x; m < M; m += gridDim.x)
-    forward_3d2d_block<float>(sm, vol + (size_t)m * kC * kVox, b2r, feat + (size_t)m * kO * kP);
 }
 
 // ---- rotate_volume materialised (refcompat) --------------------------------
@@ -288,19 +270,14 @@ int launch_score_fp32(const Scored& p, const float* tgt_feat, float* scores, cud
 
 int launch_forward_3d2d(const float* vol, const float* W1, const float* W2, const float* b2,
                         float* feat, int64_t m, cudaStream_t s) {
-  if (m == 0) return AHV_OK;
-  // the per-pair sizes of the verification step take the same kernel as the fused step's prologue, so
-  // ahv_score (caller-computed target features) and ahv_verify agree bit for bit; the persistent
-  // weight-staging kernel below serves bulk calls (refcompat: thousands of materialised volumes)
-  if (m <= 4096) return launch_tgt_feat(vol, W1, W2, b2, nullptr, feat, (int)m, s);
-  const int sms = sm_count();
-  if (sms <= 0) return AHV_ECUDA;
-  const unsigned grid = (unsigned)(m < sms ? m : sms);
-  const size_t smem = sizeof(Fp32Smem);
-  AHV_CUDA_OK(cudaFuncSetAttribute(forward_3d2d_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)smem));
-  forward_3d2d_kernel<<<grid, kThreads, smem, s>>>(vol, W1, W2, b2, feat, m);
-  AHV_CUDA_OK(cudaGetLastError());
+  // every target feature comes from the fused step's prologue kernel, whatever m is, so ahv_score (caller-computed
+  // target features), ahv_verify and the refine / search chains agree bit for bit at every batch size
+  constexpr int64_t kChunk = 1 << 30;  // launch_tgt_feat counts volumes in an int
+  for (int64_t m0 = 0; m0 < m; m0 += kChunk) {
+    const int st = launch_tgt_feat(vol + (size_t)m0 * kC * kVox, W1, W2, b2, nullptr, feat + (size_t)m0 * kO * kP,
+                                   (int)(m - m0 < kChunk ? m - m0 : kChunk), s);
+    if (st != AHV_OK) return st;
+  }
   return AHV_OK;
 }
 

@@ -207,8 +207,8 @@ int launch_typed(const Scored& p, const float* vol_tgt, const float* tgt_feat_in
 
 }  // namespace tc
 
-// forward_3d2d for B plain volumes (+ optional clear of B arg-max keys): the fused step's prologue, also
-// behind ahv_forward_3d2d for per-pair sizes
+// forward_3d2d for B plain volumes (+ optional clear of B arg-max keys): the fused step's prologue, and the one
+// kernel behind every ahv_forward_3d2d call
 int launch_tgt_feat(const float* vol_tgt, const float* W1, const float* W2, const float* b2,
                     unsigned long long* clear_keys, float* feat, int B, cudaStream_t s) {
   // same shared-memory carve-out as the scoring kernel: an SM cannot change its L1/shared split while a CTA

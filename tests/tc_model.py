@@ -18,8 +18,9 @@ operands and fp64:
   convolutions      tri-plane layout (oracle.triplane_np), D1 = W1h A in fp64, H1 = RN16(ReLU(D1)), D2 = W2h H1 in
                     fp64, D2 2^(e1+e2) / s + b2, F.normalize (eps 1e-12), dot with the target features, mean.
 
-fp32 FMA is emulated as float32(float64(a) float64(b) + float64(c)): the product is exact and the sum double-rounds
-with probability about 2^-29.  fp16 FMA the same way is exact (the sum of an fp16 product and an fp16 fits a double).
+fp32 FMA is correctly rounded: the product is exact in fp64, and the sum is rounded to odd in fp64 where rounding it
+to nearest could round twice (fma32).  fp16 FMA through fp64 is exact (the sum of an fp16 product and an fp16 fits a
+double).
 
 `rounding=False` evaluates every step in fp64 (the scorer's exact function); `rz` names sites whose fp16 conversion
 is made round-toward-zero instead ("A": the gather's output, or the staged volume of the 16-bit gather; "H1";
@@ -57,8 +58,31 @@ def rz16(x) -> np.ndarray:
 
 
 def fma32(a, b, c) -> np.ndarray:
-    """fp32 fused multiply-add, emulated through fp64 (exact product, one rounding of the sum up to double rounding)."""
-    return (np.asarray(a, f64) * np.asarray(b, f64) + np.asarray(c, f64)).astype(f32)
+    """fp32 fused multiply-add, correctly rounded.  The product of two fp32 values is exact in fp64; the sum s =
+    fl64(p + c) is made round-to-odd (TwoSum gives its error e; when e != 0 and s has an even last bit, s moves one
+    fp64 ulp towards p + c), and round-to-odd at 53 >= 2 * 24 + 2 bits followed by round-to-nearest at 24 bits is the
+    correctly rounded result (Boldo & Melquiond).  fp32 subnormal results included.
+
+    Every fp32 midpoint is an fp64 value, so RN64 cannot carry p + c across one: RN32(s) differs from RN32(p + c) only
+    when s is itself a midpoint.  Only those elements (low 29 bits 1 << 28 in the normal range) and the nonzero ones of
+    fp32's subnormal range take the round-to-odd path."""
+    p = np.asarray(a, f32).astype(f64) * np.asarray(b, f32).astype(f64)
+    c = np.asarray(c, f32).astype(f64)
+    shape = np.broadcast(p, c).shape
+    s = np.atleast_1d(p + c)
+    r = s.astype(f32)
+    u = s.view(np.int64)
+    risky = ((u & 0x1FFFFFFF) == 0x10000000) | ((np.abs(s) < 2.0 ** -126) & (s != 0))
+    if risky.any():
+        i = np.nonzero(risky)
+        pi, ci, si = np.broadcast_to(p, s.shape)[i], np.broadcast_to(c, s.shape)[i], s[i]
+        t = si - pi
+        e = (pi - (si - t)) + (ci - t)                       # TwoSum: si + e == pi + ci exactly
+        ui = si.view(np.int64)
+        fix = (e != 0) & ((ui & 1) == 0)
+        ui = ui + fix * (np.sign(e) * np.sign(si)).astype(np.int64)  # towards p + c: away from zero when e, s agree
+        r[i] = ui.view(f64).astype(f32)
+    return r.reshape(shape)
 
 
 def fma16(a, b, c) -> np.ndarray:

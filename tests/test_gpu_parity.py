@@ -411,12 +411,13 @@ def test_non_finite_inputs_do_not_hang_or_fault(ahv, golden):
     assert torch.isfinite(r.scores[0]).all() and torch.isfinite(r.scores[2]).all()
 
 
-@pytest.mark.parametrize("B,N", [(64, 3), (200, 1), (7, 2), (150, 5), (33, 17), (2, 149), (3, 296)])
+@pytest.mark.parametrize("B,N", [(64, 3), (200, 1), (7, 2), (150, 5), (33, 17), (2, 149), (3, 296), (4097, 2), (5000, 3)])
 @pytest.mark.parametrize("voldt", ["f32", "bf16"])
 def test_many_pairs_tiny_hypothesis_sets(ahv, golden, B, N, voldt):
     """Every CTA range crosses pair boundaries and most tiles are odd tails: stresses volume
     re-staging, the per-pair arg-max flush and the two-hypothesis tiling.  The fp32 CUDA-core
-    kernel (independent code path) is the on-device reference."""
+    kernel (independent code path) is the on-device reference.  Past 4096 pairs the fused call, the
+    k > 1 chain and caller-computed target features must still agree bit for bit."""
     dev = _dev()
     gen = torch.Generator().manual_seed(B * 131 + N)
     vs = (torch.randn(B, 16, 8, 8, 8, generator=gen) * 1.1 - 0.2).to(dev)
@@ -440,6 +441,9 @@ def test_many_pairs_tiny_hypothesis_sets(ahv, golden, B, N, voldt):
         assert torch.equal(multi.scores, got.scores)
         tv, _ = torch.topk(got.scores, k2, dim=1)
         assert torch.equal(multi.topk_val, tv)
+        v = ahv.HypothesisVerifier(*_weights(golden, dev))
+        given = v.score(vs, vt, R, k=1, return_scores=True, tgt_feat=v.target_features(vt))
+        assert torch.equal(given.scores, got.scores) and torch.equal(given.topk_idx, got.topk_idx)
 
 
 def test_graphed_verifier_matches_eager(ahv, golden):
