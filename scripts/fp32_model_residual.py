@@ -22,6 +22,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import fp32_model as F  # noqa: E402
+import kernel_arith as K  # noqa: E402
+import tc_model as M  # noqa: E402  (the cases)
 import test_gpu_fp32_model as G  # noqa: E402  (its inputs: rotation kinds, volumes, sizes)
 
 f32 = np.float32
@@ -36,7 +38,7 @@ def _gpu():
 def _cmp(got, want):
     got, want = np.asarray(got, f32), np.asarray(want, f32)
     same = got.view(np.uint32) == want.view(np.uint32)
-    return {"identical": float(same.mean()), "max_ulp": int(F.ulp_distance(got, want).max()), "outputs": int(same.size)}
+    return {"identical": float(same.mean()), "max_ulp": int(K.ulp_distance(got, want).max()), "outputs": int(same.size)}
 
 
 def main():
@@ -46,8 +48,8 @@ def main():
     golden = {k: dict(np.load(os.path.join(ROOT, "tests", "golden", k + ".npz"))) for k in ("weights", "shared_n3000_b3")}
     rec = {"gpu": _gpu(), "scores": {}, "target_features": {}, "rotate_volume": {}, "rotate_volume_backward": {}}
     t0 = time.time()
-    for name in F.CASES:
-        case = F.make_case(name, golden)
+    for name in M.CASES:
+        case = M.make_case(name, golden)
         head = [T(case[k]) for k in ("W1", "W2", "b2")]
         B, N = case["vs"].shape[0], case["R"].shape[-3]
         items = F.case_items(name, B, N, cap=48)
@@ -55,7 +57,7 @@ def main():
         for voldt in ("f32", "bf16"):
             v, vs = T(case["vs"]), case["vs"]
             if voldt == "bf16":
-                v, vs = v.bfloat16(), F.bf16_round(vs)
+                v, vs = v.bfloat16(), K.bf16_round(vs)
             s = ahv.ops.score(v, T(case["tgt"]), T(case["R"]), *head, k=1, math=ahv.MATH_FP32)[0]
             model = F.score(vs, case["tgt"], case["R"], case["W1"], case["W2"], case["b2"], items=items)
             row[voldt] = _cmp(s.cpu().numpy().reshape(-1)[items], model)

@@ -5,40 +5,38 @@ training forward's kept conv1 output (h1, fp16) and pair factor (pair_inv = 2^e1
 kernel to what the model leaves out - the tensor core's fp32 accumulation inside each MMA and the order of the fp32
 sums across items, CTAs and atomics, which the model takes in fp64 - instead of to 1e-3 of fp64:
 
-  fp32 gather     gather_rotated: the coordinates of make_tap (ahv_common.cuh: fmaf(R2, z, fmaf(R1, y, R0 x)), not the
-                  tensor-core scorer's order), the x-tap swap (line ^ w) & 1, corners in the (dy, dz) order, each weight
-                  wyz * wx rounded before its FMA.  tc_model.gather_f32 follows ahv_score_tc_ts.cuh instead (parity of
-                  h, other coordinate order): both restate what their kernel does.
+  fp32 gather     gather_rotated: kernel_arith.gather32 with make_tap's coordinate order fmaf(R2, z, fmaf(R1, y, R0 x))
+                  (not the tensor-core scorer's) and the x-tap swap (line ^ w) & 1 (parity="w").
   A^T operand     RN16(X * s), s = 1 / (pair_inv 2^-e1).
   packing         W1h = RN16(W1 2^-e1), W2h = RN16(W2 2^-e2) with tc_model's exponents; kappa from the fp32 column
                   L1 sums of W1h (o = 0 .. 31 in order): 2^floor(log2(2 / (3 c))).
-  conv2           v = fmaf(acc, pinv 2^e2, b2); |v|^2 and <v, T> as four 8-channel fmaf chains added as (0+1) + (2+3);
-                  the 1e-12 clamp; dH2 = (g/64) inv (T - F <F,T>), dT += (g/64) F, db2 += dH2.
+  conv2           v = fmaf(acc, pinv 2^e2, b2); |v|^2 and <v, T> by kernel_arith.head_dots; the 1e-12 clamp;
+                  dH2 = (g/64) inv (T - F <F,T>), dT += (g/64) F, db2 += dH2.
   per-item scales dH2: 2^(13 - e), e = floor(log2(2 |g/64| / max(sqrt(min_p |v_p|^2), 1e-12))) (13 when that is 0);
                   dH1: 2^(13 - e), e = floor(log2 max |dH1|) (13 when 0); both clamped to [-100, 100].
   fp16 operands   dH2h = RN16(dH2 S2), dH1h = RN16(mask (dH2h W2h) 2^(e2 - ...) S), mask = kept h1 > 0.
   dX fold         view x: RN16(acc_x kappa); views y, z: RN16(fmaf(acc, kappa, dX)) in that order (double rounding).
-  adjoint         row path: weight (wx wy) wz in fp32 -> unorm16 __float2uint_rn(w 65535), read back as
-                  float(w16) * (unscale * fp32(1/65535)); the exact path (some input voxel collects more than 16
+  adjoint         make_tap's corners; row path: weight (wx wy) wz in fp32 -> unorm16 __float2uint_rn(w 65535), read
+                  back as float(w16) * (unscale * fp32(1/65535)); the exact path (some input voxel collects more than 16
                   contributions, zero weights included) keeps the fp32 weight times unscale.
   outputs         dW1 = acc (invS pvol), dW2 = acc (inv_s2 pinv), dV = dX unscale-weighted, dT, db2.
 
-`rounding=False` evaluates every step in fp64: the exact gradient of the function the forward ran (its kept H1 and that
-value's ReLU mask).  `rz` names sites whose conversion is made round-toward-zero instead: "AT" (the A^T operand), "W1t"
-(the W1^T operand), "dH2", "dH1", "dX" (all three fold conversions), "w16" (__float2uint_rz) - the defects the gates of
-tests/test_gpu_tc_bwd_model.py must see.  `fold` is the order the three views are folded in ("xyz", as the kernel).
+The roundings, taps, gathers and head_dots are kernel_arith's.  `rounding=False` evaluates every step in fp64: the
+exact gradient of the function the forward ran (its kept H1 and that value's ReLU mask).  `rz` names sites whose
+conversion is made round-toward-zero instead: "AT" (the A^T operand), "W1t" (the W1^T operand), "dH2", "dH1", "dX"
+(all three fold conversions), "w16" (__float2uint_rz) - the defects the gates of tests/test_gpu_tc_bwd_model.py must
+see.  `fold` is the order the three views are folded in ("xyz", as the kernel).
 """
 from __future__ import annotations
-
-import os
-from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 
 import tc_model as M
+from kernel_arith import (C, KTRI, NPOS, OCH, S, VOX, exp_bits, fma32, gather32, gather64, head_dots, lattice_rotations,
+                          outside_rotations, random_rotations, random_volumes, rn16, run_chunks, rz16, sample_coords,
+                          sample_coords64, tap_at, trained_like)
 from oracle import ahv_oracle as oracle
 
-C, S, VOX, OCH, KTRI, NPOS, HALO = M.C, M.S, M.VOX, M.OCH, M.KTRI, M.NPOS, M.HALO
 LIST_CAP = 16                                                   # kListCap: contributions a row of the work list holds
 f16, f32, f64 = np.float16, np.float32, np.float64
 GRADS = ("vol_src", "tgt_feat", "W1", "W2", "b2")
@@ -47,11 +45,6 @@ GRADS = ("vol_src", "tgt_feat", "W1", "W2", "b2")
 # ---- scalar helpers -------------------------------------------------------------------------------------------------
 def _pow2(e) -> np.ndarray:
     return np.ldexp(f32(1.0), np.asarray(e, np.int64)).astype(f32)
-
-
-def exp_bits(x) -> np.ndarray:
-    """((float_as_int(x) >> 23) & 0xff) - 127: floor(log2 x) of a normal positive fp32, -127 for zero and subnormals."""
-    return ((np.asarray(x, f32).view(np.uint32) >> 23) & 0xFF).astype(np.int64) - 127
 
 
 def item_scale(m) -> tuple[np.ndarray, np.ndarray]:
@@ -90,62 +83,11 @@ def unorm16(w, rz: bool = False) -> np.ndarray:
     return (np.floor(p) if rz else np.rint(p)).astype(np.int64)
 
 
-# ---- the gather and the adjoint's taps ------------------------------------------------------------------------------
-def taps32(R: np.ndarray, base=None):
-    """make_tap of every output voxel under R [n,9] fp32: (x0, y0, z0) int [n,512] and (fx, fy, fz) fp32 [n,512]."""
-    base = oracle.base_coords_np() if base is None else np.asarray(base, f32)
-    d, h, w = M._voxels()
-    x, y, z = base[w][None], base[h][None], base[d][None]
-    u = []
-    for r in range(3):
-        R0, R1, R2 = (R[:, 3 * r + i : 3 * r + i + 1].astype(f32) for i in range(3))
-        g = M.fma32(R2, z, M.fma32(R1, y, (R0 * x).astype(f32)))
-        t = M.fma32((g + f32(1.0)).astype(f32), f32(4.0), f32(-0.5))
-        u.append(np.minimum(np.maximum(t, f32(-1.0)), f32(8.0)))
-    i0 = [np.minimum(np.floor(t), f32(7.0)) for t in u]
-    fr = [(t - a).astype(f32) for t, a in zip(u, i0)]
-    return [a.astype(np.int64) for a in i0], fr
-
-
-def taps64(R: np.ndarray, base64: np.ndarray):
-    """The same taps in fp64 from fp64 base coordinates (the exact function)."""
-    d, h, w = M._voxels()
-    p = np.stack([base64[w], base64[h], base64[d]])
-    g = np.asarray(R, f64).reshape(-1, 3, 3) @ p
-    u = np.minimum(np.maximum((g + 1.0) * 4.0 - 0.5, -1.0), 8.0)
-    i0 = np.minimum(np.floor(u), 7.0)
-    fr = u - i0
-    return [i0[:, i].astype(np.int64) for i in range(3)], [fr[:, i] for i in range(3)]
-
-
-def gather(vol: np.ndarray, slot: np.ndarray, taps, dtype, parity: bool) -> np.ndarray:
-    """Trilinear gather [n,16,512] of volumes vol [P,16,8,8,8] (item i reads vol[slot[i]]) at `taps`.  parity=True:
-    the kernel's fp32 arithmetic (lane's x-tap order (line ^ w) & 1, corners (y0,z0) (y1,z0) (y0,z1) (y1,z1), weight
-    wyz * wx rounded, then one FMA); else a plain fp64 sum."""
-    (x0, y0, z0), (fx, fy, fz) = taps
-    V, off = M._halo(vol, dtype, slot, len(slot))
-    line = ((z0 + 1) * HALO + (y0 + 1)) * HALO + (x0 + 1)
-    one = dtype(1.0)
-    swap = ((line ^ M._voxels()[2][None]) & 1) if parity else np.zeros_like(line)
-    wxa = np.where(swap == 1, fx, one - fx).astype(dtype)
-    wxb = np.where(swap == 1, one - fx, fx).astype(dtype)
-    line = line + off
-    acc = np.zeros((C,) + line.shape, dtype)
-    for c in range(4):
-        wyz = ((fy if c & 1 else one - fy) * (fz if c >> 1 else one - fz)).astype(dtype)
-        la = line + (c >> 1) * HALO * HALO + (c & 1) * HALO
-        if parity:
-            acc = M.fma32((wyz * wxa).astype(f32), V[:, la + swap], acc)
-            acc = M.fma32((wyz * wxb).astype(f32), V[:, la + 1 - swap], acc)
-        else:
-            acc = acc + wyz * wxa * V[:, la] + wyz * wxb * V[:, la + 1]
-    return acc.transpose(1, 0, 2)
-
-
+# ---- the adjoint's taps ---------------------------------------------------------------------------------------------
 def corners(taps):
     """The 8 (input voxel [n,512], inside [n,512], weight (wx wy) wz [n,512]) of every output voxel, dlt = dx + 2 dy +
     4 dz as list_pass walks them; weights in the taps' precision."""
-    (x0, y0, z0), (fx, fy, fz) = taps
+    (x0, y0, z0), (fx, fy, fz), _ = taps
     one = fx.dtype.type(1.0)
     out = []
     for dlt in range(8):
@@ -161,7 +103,7 @@ def contributions(R: np.ndarray, base=None) -> np.ndarray:
     """The largest number of contributions any input voxel collects, per matrix R [n,3,3] (the work list's row holds
     LIST_CAP; above that the item takes the exact path)."""
     R = np.asarray(R, f32).reshape(-1, 9)
-    cs = corners(taps32(R, base))
+    cs = corners(tap_at(sample_coords(R, base)))
     n = len(R)
     cnt = np.zeros((n, VOX), np.int64)
     rows = np.repeat(np.arange(n)[:, None], VOX, 1)
@@ -227,38 +169,31 @@ def tc_backward(vol_src, tgt_feat, R, W1, W2, b2, grad_scores, h1, pair_inv, *, 
         out = {"vol_src": np.zeros((len(used), C, VOX)), "tgt_feat": np.zeros((len(used), NPOS, OCH)),
                "W1": np.zeros((OCH, KTRI)), "W2": np.zeros((OCH, OCH)), "b2": np.zeros(OCH)}
         if rounding:
-            taps = taps32(Rc, base)
-            X = gather(vs[used], slot, taps, f32, True)        # [n,16,512] fp32
+            taps = tap_at(sample_coords(Rc, base))
+            X = gather32(vs[used], Rc, base, slot)             # [n,16,512] fp32
             pv = (pinv[pair] * n1).astype(f32)                 # 1/s
             sb = (f32(1.0) / pv).astype(f32)
             Xs = (X * sb[:, None, None]).astype(f32)
-            AT = (M.rz16(Xs) if "AT" in rz else M.rn16(Xs)).astype(f64)
+            AT = (rz16(Xs) if "AT" in rz else rn16(Xs)).astype(f64)
             tri = oracle.triplane_np(AT.reshape(n, C, S, S, S)).reshape(n, KTRI, NPOS)
             acc2 = np.einsum("npi,oi->npo", H, W2d).astype(f32)
-            v = M.fma32(acc2, (pinv[pair] * w2s).astype(f32)[:, None, None], b2v)      # [n,64,32] fp32
-            vq, tq = v.reshape(n, NPOS, 4, 8), tgp.reshape(n, NPOS, 4, 8)
-            ss = np.zeros((n, NPOS, 4), f32)
-            ft = np.zeros((n, NPOS, 4), f32)
-            for oo in range(8):
-                ss = M.fma32(vq[..., oo], vq[..., oo], ss)
-                ft = M.fma32(vq[..., oo], tq[..., oo], ft)
-            ss = (ss[..., 0] + ss[..., 1]) + (ss[..., 2] + ss[..., 3])
-            ft = (ft[..., 0] + ft[..., 1]) + (ft[..., 2] + ft[..., 3])
+            v = fma32(acc2, (pinv[pair] * w2s).astype(f32)[:, None, None], b2v)      # [n,64,32] fp32
+            ss, ft = head_dots(v, tgp)
             nraw = np.sqrt(ss)
             inv = (f32(1.0) / np.maximum(nraw, f32(1e-12))).astype(f32)[..., None]
             fdot = (ft[..., None] * inv).astype(f32)
             g64 = (g_item * f32(1.0 / 64.0)).astype(f32)[:, None, None]
             F = (v * inv).astype(f32)
-            par = np.where((nraw < f32(1e-12))[..., None], tgp, M.fma32(-F, fdot, tgp))
+            par = np.where((nraw < f32(1e-12))[..., None], tgp, fma32(-F, fdot, tgp))
             d2 = ((g64 * inv).astype(f32) * par).astype(f32)
             S2, inv_s2 = item_scale(dh2_bound(g64[:, 0, 0], ss.min(axis=1)))
             p2 = (d2 * S2[:, None, None]).astype(f32)
-            dH2h = (M.rz16(p2) if "dH2" in rz else M.rn16(p2)).astype(f64)
+            dH2h = (rz16(p2) if "dH2" in rz else rn16(p2)).astype(f64)
             accH1 = np.einsum("npo,oi->npi", dH2h, W2d).astype(f32)
             dh1 = np.where(H > 0, (accH1 * (inv_s2 * w2s).astype(f32)[:, None, None]).astype(f32), f32(0.0))
             Sd, invS = item_scale(np.abs(dh1).max(axis=(1, 2)))
             p1 = (dh1 * Sd[:, None, None]).astype(f32)
-            dH1h = (M.rz16(p1) if "dH1" in rz else M.rn16(p1)).astype(f64)
+            dH1h = (rz16(p1) if "dH1" in rz else rn16(p1)).astype(f64)
             accW2 = np.einsum("npo,npi->noi", dH2h, H).astype(f32)
             out["W2"] += np.einsum("noi,n->oi", accW2.astype(f64), (inv_s2 * pinv[pair]).astype(f32).astype(f64))
             accW1 = np.einsum("npo,nkp->nok", dH1h, tri).astype(f32)
@@ -267,8 +202,8 @@ def tc_backward(vol_src, tgt_feat, R, W1, W2, b2, grad_scores, h1, pair_inv, *, 
             dX = None
             for vname in fold:
                 a = views[vname].reshape(n, C, VOX)
-                p = (a * kappa).astype(f32) if dX is None else M.fma32(a, kappa, dX)
-                dX = (M.rz16(p) if "dX" in rz else M.rn16(p)).astype(f32)
+                p = (a * kappa).astype(f32) if dX is None else fma32(a, kappa, dX)
+                dX = (rz16(p) if "dX" in rz else rn16(p)).astype(f32)
             unscale = (invS * inv_kappa).astype(f32)
             cs = corners(taps)
             cnt = np.zeros((n, VOX), np.int64)
@@ -285,8 +220,8 @@ def tc_backward(vol_src, tgt_feat, R, W1, W2, b2, grad_scores, h1, pair_inv, *, 
             dT = g64.astype(f64) * F.astype(f64)
             dX = dX.astype(f64)
         else:
-            taps = taps64(Rc, base64)
-            X = gather(vs[used].astype(f64), slot, taps, f64, False)
+            taps = tap_at(sample_coords64(Rc, base64))
+            X = gather64(vs[used], Rc, base64, slot)
             tri = oracle.triplane_np(X.reshape(n, C, S, S, S)).reshape(n, KTRI, NPOS)
             Ht = H * pinv[pair].astype(f64)[:, None, None]
             v = np.einsum("npi,oi->npo", Ht, W2d) + b2v.astype(f64)
@@ -318,16 +253,13 @@ def tc_backward(vol_src, tgt_feat, R, W1, W2, b2, grad_scores, h1, pair_inv, *, 
     res = {"vol_src": np.zeros((B, C, VOX)), "tgt_feat": np.zeros((B, NPOS, OCH)), "W1": np.zeros((OCH, KTRI)),
            "W2": np.zeros((OCH, OCH)), "b2": np.zeros(OCH)}
     exact, count = np.zeros(B * N, bool), np.zeros(B * N, np.int64)
-    # numpy releases the GIL in its loops: chunks of items run on all cores; their sums are added in chunk order
-    with ThreadPoolExecutor(max_workers=os.cpu_count() or 1) as pool:
-        starts = list(range(0, B * N, chunk))
-        for i0, fut in zip(starts, [pool.submit(run, i0) for i0 in starts]):
-            used, out, ex, cn = fut.result()
-            res["vol_src"][used] += out["vol_src"]
-            res["tgt_feat"][used] += out["tgt_feat"]
-            for k in ("W1", "W2", "b2"):
-                res[k] += out[k]
-            exact[i0 : i0 + len(ex)], count[i0 : i0 + len(cn)] = ex, cn
+    starts = range(0, B * N, chunk)
+    for i0, (used, out, ex, cn) in zip(starts, run_chunks(run, starts)):    # the chunks' sums added in chunk order
+        res["vol_src"][used] += out["vol_src"]
+        res["tgt_feat"][used] += out["tgt_feat"]
+        for k in ("W1", "W2", "b2"):
+            res[k] += out[k]
+        exact[i0 : i0 + len(ex)], count[i0 : i0 + len(cn)] = ex, cn
     grads = {"vol_src": res["vol_src"].reshape(B, C, S, S, S), "tgt_feat": res["tgt_feat"].transpose(0, 2, 1).copy(),
              "W1": res["W1"], "W2": res["W2"], "b2": res["b2"]}
     if info:
@@ -364,20 +296,6 @@ GATE = {"vol_src": {"elem": 7.5e-4, "l2": 1.5e-4}, "tgt_feat": {"elem": 2e-6, "l
 
 
 # ---- the cases tests/test_gpu_tc_bwd_model.py and scripts/tc_bwd_model_residual.py run -------------------------------
-def axis_rotation(axis, deg) -> np.ndarray:
-    a = np.asarray(axis, f64) / np.linalg.norm(axis)
-    t = np.deg2rad(deg)
-    K = np.array([[0, -a[2], a[1]], [a[2], 0, -a[0]], [-a[1], a[0], 0]])
-    return (np.eye(3) + np.sin(t) * K + (1 - np.cos(t)) * K @ K).astype(f32)
-
-
-def outside_rotations() -> np.ndarray:
-    """Rotations that send samples outside [-1, 8): 45 degrees about z, 30 about a face diagonal, and three more (the
-    set of tests/test_gpu_rotation_grad.py)."""
-    return np.stack([axis_rotation((0, 0, 1), 45), axis_rotation((1, 1, 0), 30), axis_rotation((1, 0, 0), 45),
-                     axis_rotation((0, 1, 1), 60), axis_rotation((1, -2, 0.5), 135)])
-
-
 CASES = (["golden"]
          + ["shape_1x1", "shape_1x3", "shape_3x49_per_pair", "shape_300x3", "shape_12x400_per_pair"]
          + ["lattice", "outside", "R_x0.35", "R_mixed_x0.35"]
@@ -402,17 +320,17 @@ def make_case(name: str, golden: dict) -> dict:
     elif name.startswith("shape_"):
         B, N = map(int, name.split("_")[1].split("x"))
         per_pair = name.endswith("per_pair")
-        vs, vt = M._vols(rng, B)
+        vs, vt = random_volumes(rng, B)
     elif name == "lattice":
-        B, R = 2, M.lattice_rotations()
+        B, R = 2, lattice_rotations()
     elif name == "outside":
-        R = np.concatenate([outside_rotations(), M._rot(rng, 60)])
+        R = np.concatenate([outside_rotations(), random_rotations(rng, 60)])
     elif name == "R_x0.35":                                   # not rotations: every item takes the exact path
         B, N = 2, 150
-        R = (M._rot(rng, N) * f32(0.35)).astype(f32)
+        R = (random_rotations(rng, N) * f32(0.35)).astype(f32)
     elif name == "R_mixed_x0.35":                             # every fifth matrix shrunk: the path changes per item
         B, N = 2, 150
-        R = M._rot(rng, B, N)
+        R = random_rotations(rng, B, N)
         R[:, ::5] *= f32(0.35)
     elif name.startswith("vol_x"):
         vs = (np.asarray(vs) * f32(float(name[5:]))).astype(f32)
@@ -428,12 +346,12 @@ def make_case(name: str, golden: dict) -> dict:
     elif name == "W2_x0.05":
         W2 = (W2 * f32(0.05)).astype(f32)
     elif name in ("student_t", "row_scales", "zero_rows"):
-        W1, W2 = M._trained_like(W1, W2, name, seed=77)
+        W1, W2 = trained_like(W1, W2, name, seed=77)
     elif name == "zero_conv2":                                # H2 = 0 everywhere: the normalisation's clamp
         tgt_w = (W1, W2, b2)
         W2, b2 = np.zeros_like(W2), np.zeros_like(b2)
     if R is None:
-        R = M._rot(rng, B, N) if per_pair else M._rot(rng, N)
+        R = random_rotations(rng, B, N) if per_pair else random_rotations(rng, N)
     N = R.shape[-3]
     vs = np.ascontiguousarray(np.asarray(vs)[:B], f32)
     vt = np.ascontiguousarray(np.asarray(vt)[:B], f32)
@@ -488,8 +406,8 @@ def fp64_autograd(vs, tgt, R, W1, W2, b2, gs, h1, pair_inv, want_R: bool = False
 
 def r_set(B, N, per_pair, seed):
     """Random rotations with the 24 lattice rotations and the out-of-range ones mixed in (evenly spaced)."""
-    special = np.concatenate([M.lattice_rotations(), outside_rotations()])
-    R = M._rot(np.random.default_rng(seed), *((B, N) if per_pair else (N,)))
+    special = np.concatenate([lattice_rotations(), outside_rotations()])
+    R = random_rotations(np.random.default_rng(seed), *((B, N) if per_pair else (N,)))
     flat = R.reshape(-1, 3, 3)
     step = max(1, flat.shape[0] // len(special))
     k = len(flat[::step][: len(special)])

@@ -9,18 +9,17 @@ operands and fp64:
                     (lane partial sums over columns lane + 32 j, then the xor butterfly 16, 8, 4, 2, 1);
                     W1h = RN16(W1 2^-e1), W2h = RN16(W2 2^-e2), fp16 subnormals included.
   pair scale        stage_pair_volume: bound = min(8192, 32768 / l1n), e = ilogb(bound / max|V|) in [-100, 100].
-  fp32 gather       the kernel's coordinate FMAs, clamp and floor, the lane's x-tap order (bank parity of the
-                    line), y-z corners in the order (y0,z0) (y1,z0) (y0,z1) (y1,z1), each corner weight rounded to
-                    fp32 before its FMA; then RN16.
+  fp32 gather       kernel_arith.gather32 with the scorer's own coordinate order fmaf(R0, x, fmaf(R2, z, R1 y))
+                    (coords="tc") and the x taps swapped by the bank parity (h >> 2) & 1 of the lane (parity="h"),
+                    not w as gather_hypothesis; then RN16.
   16-bit gather     staged volume RN16(V s); fp16 weights and their fp16 products; per channel 8 fp16 FMAs, first x
                     tap (rot >> 1) then the other, corners (ya,z0) (ya,z1) (yb,z0) (yb,z1), ya = the y tap whose
-                    x-pair line has the lane's bank parity.
+                    x-pair line has the lane's bank parity; taps as the fp32 gather's.
   convolutions      tri-plane layout (oracle.triplane_np), D1 = W1h A in fp64, H1 = RN16(ReLU(D1)), D2 = W2h H1 in
                     fp64, D2 2^(e1+e2) / s + b2, F.normalize (eps 1e-12), dot with the target features, mean.
 
-fp32 FMA is correctly rounded: the product is exact in fp64, and the sum is rounded to odd in fp64 where rounding it
-to nearest could round twice (fma32).  fp16 FMA through fp64 is exact (the sum of an fp16 product and an fp16 fits a
-double).
+The steps this kernel shares with others (roundings, taps, the fp32 and fp64 gathers, the halo layout, the butterfly)
+are kernel_arith's.
 
 `rounding=False` evaluates every step in fp64 (the scorer's exact function); `rz` names sites whose fp16 conversion
 is made round-toward-zero instead ("A": the gather's output, or the staged volume of the 16-bit gather; "H1";
@@ -28,74 +27,18 @@ is made round-toward-zero instead ("A": the gather's output, or the staged volum
 """
 from __future__ import annotations
 
-import os
-from concurrent.futures import ThreadPoolExecutor
-
 import numpy as np
 
+from kernel_arith import (C, HALO, KTRI, NPOS, OCH, S, VOX, bf16_round, butterfly, fma16, gather32, gather64, halo,
+                          ilogb32, lattice_rotations, random_rotations, random_volumes, rn16, run_chunks, rz16,
+                          sample_coords, tap_at, trained_like, voxels)
 from oracle import ahv_oracle as oracle
 
-C, S, VOX, OCH, KTRI, NPOS = 16, 8, 512, 32, 384, 64
-HALO = 10
 W1_NORM_TARGET, W2_NORM_TARGET = 2, 0          # ahv_common.cuh kW1NormTarget, kW2NormTarget
 f32, f64, f16 = np.float32, np.float64, np.float16
 
 
-# ---- scalar helpers -------------------------------------------------------------------------------------------------
-def rn16(x) -> np.ndarray:
-    """Round to fp16, to nearest even, subnormals and overflow to inf included (cvt.rn.f16)."""
-    with np.errstate(over="ignore"):
-        return np.asarray(x).astype(f16)
-
-
-def rz16(x) -> np.ndarray:
-    """Round to fp16 toward zero (cvt.rz.f16): finite inputs never become inf."""
-    x = np.asarray(x, dtype=f64)
-    with np.errstate(over="ignore"):
-        h = x.astype(f16)
-    over = np.abs(h.astype(f64)) > np.abs(x)
-    return np.where(over, np.nextafter(h, f16(0)), h)
-
-
-def fma32(a, b, c) -> np.ndarray:
-    """fp32 fused multiply-add, correctly rounded.  The product of two fp32 values is exact in fp64; the sum s =
-    fl64(p + c) is made round-to-odd (TwoSum gives its error e; when e != 0 and s has an even last bit, s moves one
-    fp64 ulp towards p + c), and round-to-odd at 53 >= 2 * 24 + 2 bits followed by round-to-nearest at 24 bits is the
-    correctly rounded result (Boldo & Melquiond).  fp32 subnormal results included.
-
-    Every fp32 midpoint is an fp64 value, so RN64 cannot carry p + c across one: RN32(s) differs from RN32(p + c) only
-    when s is itself a midpoint.  Only those elements (low 29 bits 1 << 28 in the normal range) and the nonzero ones of
-    fp32's subnormal range take the round-to-odd path."""
-    p = np.asarray(a, f32).astype(f64) * np.asarray(b, f32).astype(f64)
-    c = np.asarray(c, f32).astype(f64)
-    shape = np.broadcast(p, c).shape
-    s = np.atleast_1d(p + c)
-    r = s.astype(f32)
-    u = s.view(np.int64)
-    risky = ((u & 0x1FFFFFFF) == 0x10000000) | ((np.abs(s) < 2.0 ** -126) & (s != 0))
-    if risky.any():
-        i = np.nonzero(risky)
-        pi, ci, si = np.broadcast_to(p, s.shape)[i], np.broadcast_to(c, s.shape)[i], s[i]
-        t = si - pi
-        e = (pi - (si - t)) + (ci - t)                       # TwoSum: si + e == pi + ci exactly
-        ui = si.view(np.int64)
-        fix = (e != 0) & ((ui & 1) == 0)
-        ui = ui + fix * (np.sign(e) * np.sign(si)).astype(np.int64)  # towards p + c: away from zero when e, s agree
-        r[i] = ui.view(f64).astype(f32)
-    return r.reshape(shape)
-
-
-def fma16(a, b, c) -> np.ndarray:
-    """fp16 fused multiply-add (HFMA2): exact in fp64, rounded once to fp16."""
-    return rn16(np.asarray(a, f64) * np.asarray(b, f64) + np.asarray(c, f64))
-
-
-def ilogb32(x) -> np.ndarray:
-    """ilogbf of positive float32 values: floor(log2 x), subnormals included, INT_MAX for inf."""
-    x = np.asarray(x, f32)
-    return np.where(np.isinf(x), 2**31 - 1, np.frexp(x)[1].astype(np.int64) - 1)
-
-
+# ---- packing and the pair scale --------------------------------------------------------------------------------------
 def row_l1max(W: np.ndarray) -> f32:
     """row_l1max (ahv_common.cuh): each row's L1 norm in fp32 - lane l sums |W[r, l + 32 j]| over j, then the xor
     butterfly adds lanes 16, 8, 4, 2, 1 apart - and the largest of them."""
@@ -104,10 +47,7 @@ def row_l1max(W: np.ndarray) -> f32:
     part = np.zeros((rows, 32), f32)
     for j in range(cols // 32):
         part = (part + W[:, 32 * j : 32 * j + 32]).astype(f32)
-    lane = np.arange(32)
-    for o in (16, 8, 4, 2, 1):
-        part = (part + part[:, lane ^ o]).astype(f32)
-    return f32(part[:, 0].max())
+    return f32(butterfly(part).max())
 
 
 def weight_exponent(l1max, target: int) -> int:
@@ -129,83 +69,11 @@ def pair_exponent(l1max, vmax) -> int | None:
     return int(max(-100, min(100, int(ilogb32(q)))))
 
 
-# ---- coordinates ----------------------------------------------------------------------------------------------------
-def _voxels():
-    v = np.arange(VOX)
-    return v >> 6, (v >> 3) & 7, v & 7                       # (d, h, w) of the output voxel
-
-
-def _coords32(R: np.ndarray, base: np.ndarray):
-    """[n,9] fp32 -> clamped (ix, iy, iz) [n,512] fp32 exactly as the gather computes them:
-    fmaf(R0, bx, fmaf(R2, bz, R1 by)), unnorm = fmaf(g + 1, 4, -0.5), clamp to [-1, 8]."""
-    d, h, w = _voxels()
-    bx, by, bz = base[w][None], base[h][None], base[d][None]
-    out = []
-    for r in range(3):
-        R0, R1, R2 = (R[:, 3 * r + i : 3 * r + i + 1].astype(f32) for i in range(3))
-        pg = fma32(R2, bz, (R1 * by).astype(f32))
-        g = fma32(R0, bx, pg)
-        u = fma32((g + f32(1.0)).astype(f32), f32(4.0), f32(-0.5))
-        out.append(np.minimum(np.maximum(u, f32(-1.0)), f32(8.0)))
-    return out
-
-
-def _coords64(R: np.ndarray, base: np.ndarray):
-    d, h, w = _voxels()
-    b = base.astype(f64)
-    p = np.stack([b[w], b[h], b[d]])                         # [3,512]
-    g = R.reshape(-1, 3, 3).astype(f64) @ p                  # [n,3,512]
-    u = (g + 1.0) * 4.0 - 0.5
-    return [np.minimum(np.maximum(u[:, i], -1.0), 8.0) for i in range(3)]
-
-
-def _halo(vol: np.ndarray, dtype, pair, n: int):
-    """[P,16,8,8,8] or [16,8,8,8] -> ([16, P*1000] with the zero halo: line ((z+1)*10 + (y+1))*10 + (x+1) of volume p
-    at p*1000 + line, the line offset [n,1] of each hypothesis' volume)."""
-    vol = np.asarray(vol).reshape(-1, C, S, S, S)
-    out = np.zeros((vol.shape[0], C, HALO, HALO, HALO), dtype)
-    out[:, :, 1:9, 1:9, 1:9] = vol
-    off = np.zeros((n, 1), np.int64) if pair is None else np.asarray(pair, np.int64).reshape(n, 1) * HALO ** 3
-    return out.transpose(1, 0, 2, 3, 4).reshape(C, -1), off
-
-
-# ---- gathers --------------------------------------------------------------------------------------------------------
-def gather_f32(vs: np.ndarray, R: np.ndarray, base=None, pair=None) -> np.ndarray:
-    """The fp32 gather of an fp32 volume [16,8,8,8] (already scaled) under R [n,3,3]: [n,16,512] fp32, before RN16.
-    With volumes [P,16,8,8,8], hypothesis i samples volume pair[i]."""
-    base = oracle.base_coords_np() if base is None else np.asarray(base, f32)
-    R = np.asarray(R, f32).reshape(-1, 9)
-    ix, iy, iz = _coords32(R, base)
-    x0, y0, z0 = (np.minimum(np.floor(t), f32(7.0)) for t in (ix, iy, iz))
-    fx, fy, fz = (ix - x0).astype(f32), (iy - y0).astype(f32), (iz - z0).astype(f32)
-    x0, y0, z0 = (t.astype(np.int64) for t in (x0, y0, z0))
-    line = ((z0 + 1) * HALO + (y0 + 1)) * HALO + (x0 + 1)
-    h = _voxels()[1]
-    pf = (h >> 2) & 1                                        # bank parity this lane reads first
-    swap = (line ^ pf[None]) & 1
-    one = f32(1.0)
-    wxa = np.where(swap == 1, fx, one - fx).astype(f32)
-    wxb = np.where(swap == 1, one - fx, fx).astype(f32)
-    V, off = _halo(vs, f32, pair, len(R))
-    line = line + off
-    acc = np.zeros((C,) + line.shape, f32)
-    for c in range(4):
-        wyz = ((fy if c & 1 else one - fy).astype(f32) * (fz if c >> 1 else one - fz).astype(f32)).astype(f32)
-        la = line + (c >> 1) * HALO * HALO + (c & 1) * HALO
-        acc = fma32((wyz * wxa).astype(f32), V[:, la + swap], acc)
-        acc = fma32((wyz * wxb).astype(f32), V[:, la + 1 - swap], acc)
-    return acc.transpose(1, 0, 2)
-
-
+# ---- the 16-bit gather -----------------------------------------------------------------------------------------------
 def gather_f16(vh: np.ndarray, R: np.ndarray, base=None, pair=None) -> np.ndarray:
-    """The 16-bit gather of a staged fp16 volume [16,8,8,8] under R [n,3,3]: [n,16,512] fp16 (volumes as gather_f32)."""
-    base = oracle.base_coords_np() if base is None else np.asarray(base, f32)
-    R = np.asarray(R, f32).reshape(-1, 9)
-    ix, iy, iz = _coords32(R, base)
-    x0, y0, z0 = (np.minimum(np.floor(t), f32(7.0)) for t in (ix, iy, iz))
-    fx, fy, fz = (ix - x0).astype(f32), (iy - y0).astype(f32), (iz - z0).astype(f32)
-    x0, y0, z0 = (t.astype(np.int64) for t in (x0, y0, z0))
-    d, h, _ = _voxels()
+    """The 16-bit gather of a staged fp16 volume [16,8,8,8] under R [n,3,3]: [n,16,512] fp16 (volumes as gather32)."""
+    (x0, y0, z0), (fx, fy, fz), _ = tap_at(sample_coords(R, base, coords="tc"))
+    d, h, _ = voxels()
     pf = ((h >> 2) & 1)[None]
     rot = (((h & 3) + (d & 1)) & 3)[None]
     pline = ((z0 + 1) * HALO + (y0 + 1)) * 9 + (x0 + 1)      # x-pair line: taps x0, x0 + 1
@@ -217,7 +85,7 @@ def gather_f16(vh: np.ndarray, R: np.ndarray, base=None, pair=None) -> np.ndarra
     wz = (rn16(one - fz), rn16(fz))
     tx = (x0 + (rot >> 1), x0 + 1 - (rot >> 1))
     ty = (y0 + swapy, y0 + 1 - swapy)
-    V, off = _halo(vh, f16, pair, len(R))
+    V, off = halo(vh, f16, pair, len(x0))
     acc = np.zeros((C,) + fx.shape, f16)
     for t in range(2):
         for a in range(2):
@@ -225,24 +93,6 @@ def gather_f16(vh: np.ndarray, R: np.ndarray, base=None, pair=None) -> np.ndarra
                 wg = rn16(wx[t].astype(f64) * rn16(wy[a].astype(f64) * wz[b]).astype(f64))
                 lin = ((z0 + b + 1) * HALO + (ty[a] + 1)) * HALO + (tx[t] + 1) + off
                 acc = fma16(wg, V[:, lin], acc)
-    return acc.transpose(1, 0, 2)
-
-
-def gather_f64(vs: np.ndarray, R: np.ndarray, base=None, pair=None) -> np.ndarray:
-    """Trilinear resampling with zero padding in fp64 (no rounding anywhere): [n,16,512] fp64."""
-    base = oracle.base_coords_np() if base is None else np.asarray(base, f32)
-    R = np.asarray(R, f32).reshape(-1, 9)
-    ix, iy, iz = _coords64(R, base)
-    x0, y0, z0 = (np.minimum(np.floor(t), 7.0) for t in (ix, iy, iz))
-    fx, fy, fz = ix - x0, iy - y0, iz - z0
-    x0, y0, z0 = (t.astype(np.int64) for t in (x0, y0, z0))
-    V, off = _halo(np.asarray(vs, f64), f64, pair, len(R))
-    acc = np.zeros((C,) + fx.shape, f64)
-    for dz in (0, 1):
-        for dy in (0, 1):
-            for dx in (0, 1):
-                wgt = (fx if dx else 1 - fx) * (fy if dy else 1 - fy) * (fz if dz else 1 - fz)
-                acc += wgt * V[:, ((z0 + dz + 1) * HALO + (y0 + dy + 1)) * HALO + (x0 + dx + 1) + off]
     return acc.transpose(1, 0, 2)
 
 
@@ -303,11 +153,11 @@ def tc_forward(vol_src, tgt_feat, R, W1, W2, b2, *, gather: str = "f32", roundin
         Rc = Rall[items if per_pair else items % N]
         used, slot = np.unique(pair, return_inverse=True)      # the chunk's volumes only
         if not rounding:
-            A = gather_f64(staged[used], Rc, base, slot)
+            A = gather64(staged[used], Rc, base, slot)
         elif gather == "f16":
             A = gather_f16(staged[used], Rc, base, slot).astype(f64)
         else:
-            g = gather_f32(staged[used], Rc, base, slot)
+            g = gather32(staged[used], Rc, base, slot, parity="h", coords="tc")
             A = (rz16(g) if "A" in rz else rn16(g)).astype(f64)
         tri = oracle.triplane_np(A.reshape(-1, C, S, S, S)).reshape(-1, KTRI, NPOS)
         H1 = np.maximum(W1d @ tri, 0.0)
@@ -320,10 +170,7 @@ def tc_forward(vol_src, tgt_feat, R, W1, W2, b2, *, gather: str = "f32", roundin
             h1[items] = H1.transpose(0, 2, 1).astype(f16)
             bound[items] = (np.abs(W1d) @ np.abs(tri)).transpose(0, 2, 1)
 
-    # numpy releases the GIL in its loops: chunks of items run on all cores
-    with ThreadPoolExecutor(max_workers=os.cpu_count() or 1) as pool:
-        for fut in [pool.submit(run, i0) for i0 in range(0, B * N, chunk)]:
-            fut.result()
+    run_chunks(run, range(0, B * N, chunk))
     if want_h1:
         return scores, h1, pair_inv, bound
     return scores
@@ -348,52 +195,6 @@ def gate(mode: str, case: str) -> float:
 MODES = {"tc": "f32", "f16gather": "f16", "bf16": "f16"}     # mode -> the gather it runs
 
 
-def bf16_round(x: np.ndarray) -> np.ndarray:
-    """float32 -> the float32 value of its bf16 rounding (to nearest even), as torch's .bfloat16() makes it."""
-    u = np.ascontiguousarray(x, f32).view(np.uint32).astype(np.uint64)
-    u = ((u + 0x7FFF + ((u >> 16) & 1)) >> 16) << 16
-    return u.astype(np.uint32).view(f32)
-
-
-def lattice_rotations() -> np.ndarray:
-    """The 24 proper signed permutation matrices [24,3,3]: every sample lands on a lattice point."""
-    import itertools
-
-    out = []
-    for p in itertools.permutations(range(3)):
-        for sg in itertools.product((1, -1), repeat=3):
-            R = np.zeros((3, 3), f32)
-            R[[0, 1, 2], list(p)] = sg
-            if np.linalg.det(R) > 0:
-                out.append(R)
-    return np.stack(out)
-
-
-def _rot(rng, *shape):
-    n = int(np.prod(shape))
-    return oracle.rotations_from_normals_np(rng.normal(size=(n, 4)).astype(f32)).reshape(*shape, 3, 3)
-
-
-def _vols(rng, B):
-    return [(rng.normal(size=(B, C, S, S, S)) * 1.1 - 0.2).astype(f32) for _ in range(2)]
-
-
-def _trained_like(W1, W2, kind, seed):
-    """tests/test_gpu_weight_range.py's kinds of trained-looking head weights, drawn with numpy."""
-    rng = np.random.default_rng(seed)
-    if kind == "row_scales":                                 # log-uniform row scales over 2^0 .. 2^6
-        W1 = W1 * np.exp2(rng.random((OCH, 1)) * 6)
-    elif kind == "student_t":                                # heavy-tailed entries (df = 3), about 10 % exact zeros
-        def draw(shape, scale):
-            t = rng.normal(size=shape) / np.sqrt((rng.normal(size=(3,) + shape) ** 2).sum(0) / 3)
-            return np.where(rng.random(shape) < 0.1, 0.0, t * scale)
-        W1, W2 = draw((OCH, KTRI), 1 / np.sqrt(KTRI)), draw((OCH, OCH), 1 / np.sqrt(OCH))
-    elif kind == "zero_rows":                                # two dead conv1 channels
-        W1 = W1.copy()
-        W1[[5, 22]] = 0.0
-    return W1.astype(f32), W2.astype(f32)
-
-
 CASES = (["golden"]
          + [f"ragged_{B}x{N}_{r}" for B, N in ((1, 1), (1, 7), (2, 33), (5, 1000)) for r in ("shared", "per_pair")]
          + ["pairs_150x5", "pairs_33x17", "pairs_2400x1_mixed"]
@@ -414,44 +215,44 @@ def make_case(name: str, golden: dict) -> dict:
         R = g["R"]
     elif name.startswith("ragged_"):
         B, N = map(int, name.split("_")[1].split("x"))
-        vs, vt = _vols(rng, B)
-        R = _rot(rng, B, N) if name.endswith("per_pair") else _rot(rng, N)
+        vs, vt = random_volumes(rng, B)
+        R = random_rotations(rng, B, N) if name.endswith("per_pair") else random_rotations(rng, N)
     elif name.startswith("pairs_"):
         B, N = map(int, name.split("_")[1].split("x"))
-        vs, vt = _vols(rng, B)
-        R = _rot(rng, B, N)
+        vs, vt = random_volumes(rng, B)
+        R = random_rotations(rng, B, N)
         if name.endswith("mixed"):                           # pair magnitudes over eight decades
             vs = (vs * (10.0 ** rng.uniform(-4, 4, (B, 1, 1, 1, 1)))).astype(f32)
     elif name == "lattice":
         R = lattice_rotations()
     elif name == "beyond_volume":                            # rotations scaled by 2.5: most samples land outside
-        R = (_rot(rng, 300) * f32(2.5)).astype(f32)
+        R = (random_rotations(rng, 300) * f32(2.5)).astype(f32)
     elif name == "R_x0.35":                                  # a zoom into the centre: taps of fine fractional weight
-        R = (_rot(rng, 300) * f32(0.35)).astype(f32)
+        R = (random_rotations(rng, 300) * f32(0.35)).astype(f32)
     elif name.startswith("vol_x"):
         c = f32(float(name[5:]))
-        vs, vt = _vols(rng, 3)
+        vs, vt = random_volumes(rng, 3)
         vs = (vs * c).astype(f32)
-        R = _rot(rng, 300)
+        R = random_rotations(rng, 300)
     elif name.startswith("outlier_"):                        # standard-normal bulk, outliers +r/3 and -r
         r = float(name[8:])
         B = 3
         vs = rng.normal(size=(B, C * VOX)).astype(f32)
-        vt = _vols(rng, B)[1]
+        vt = random_volumes(rng, B)[1]
         for b in range(B):
             p = rng.permutation(C * VOX)[:2]
             vs[b, p[0]], vs[b, p[1] if b else 0] = r / 3, -r
         vs = vs.reshape(B, C, S, S, S)
-        R = _rot(rng, 300)
+        R = random_rotations(rng, 300)
     elif name.startswith("W1_x"):
         c = 2.0 ** int(name[6:]) if "^" in name else float(name[4:])
         W1 = (W1 * f32(c)).astype(f32)
         if c < 1:                                            # b2 along, or the bias alone would decide the score
             b2 = (b2 * f32(c)).astype(f32)
-        R = _rot(rng, 300)
+        R = random_rotations(rng, 300)
     else:
-        W1, W2 = _trained_like(W1, W2, name, seed=77)
-        R = _rot(rng, 300)
+        W1, W2 = trained_like(W1, W2, name, seed=77)
+        R = random_rotations(rng, 300)
     vs, vt = np.ascontiguousarray(vs, f32), np.ascontiguousarray(vt, f32)
     tgt = g["tgt_feat"] if name == "golden" else oracle.forward_3d2d_np(vt, W1, W2, b2)
     return dict(vs=vs, vt=vt, R=np.ascontiguousarray(R, f32), W1=W1, W2=W2, b2=b2, tgt=np.ascontiguousarray(tgt, f32))

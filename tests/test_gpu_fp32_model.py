@@ -23,6 +23,8 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import fp32_model as F  # noqa: E402  (tests/fp32_model.py)
+import kernel_arith as K  # noqa: E402
+import tc_model as M  # noqa: E402  (the cases)
 
 pytestmark = pytest.mark.gpu
 DEV = torch.device("cuda", 0)
@@ -44,7 +46,7 @@ def _bits_report(got, want, where):
     if same.all():
         return ""
     bad = np.argwhere(~same)
-    ulps = F.ulp_distance(got, want)
+    ulps = K.ulp_distance(got, want)
     return (f"{len(bad)} of {same.size} differ, at most {int(ulps.max())} ulps; first: "
             + ", ".join(f"{where(tuple(int(i) for i in b))} {int(ulps[tuple(b)])} ulp" for b in bad[:6]))
 
@@ -57,12 +59,12 @@ def case(golden, request):
     name = request.param
     if name not in _CASES:
         _CASES.clear()
-        _CASES[name] = dict(F.make_case(name, golden), name=name)
+        _CASES[name] = dict(M.make_case(name, golden), name=name)
     return _CASES[name]
 
 
 # ---- the scorer -----------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("case", F.CASES, indirect=True)
+@pytest.mark.parametrize("case", M.CASES, indirect=True)
 @pytest.mark.parametrize("voldt", ["f32", "bf16"])
 def test_fp32_scores_bit_identical_to_the_model(ahv, case, voldt):
     """ahv_score under AHV_MATH_FP32 runs the whole case; the model scores the golden set's first 200 hypotheses of
@@ -70,7 +72,7 @@ def test_fp32_scores_bit_identical_to_the_model(ahv, case, voldt):
     vs = case["vs"]
     v = _T(vs)
     if voldt == "bf16":
-        v, vs = v.bfloat16(), F.bf16_round(vs)
+        v, vs = v.bfloat16(), K.bf16_round(vs)
     R = case["R"]
     B, N = vs.shape[0], R.shape[-3]
     s, _, _ = ahv.ops.score(v, _T(case["tgt"]), _T(R), *_head(case), k=min(4, N), math=ahv.MATH_FP32)
@@ -112,9 +114,9 @@ def test_target_features_bit_identical_to_the_model(ahv, golden, many_volumes, m
 # ---- rotate_volume --------------------------------------------------------------------------------------------------
 def _rotations(kind: str, n: int, seed: int) -> np.ndarray:
     rng = np.random.default_rng(seed)
-    R = F.T._rot(rng, n)
+    R = K.random_rotations(rng, n)
     if kind == "lattice":
-        L = F.lattice_rotations()
+        L = K.lattice_rotations()
         R = L[np.arange(n) % len(L)]
     elif kind == "beyond_volume":                            # most samples land outside the volume
         R = R * f32(2.5)

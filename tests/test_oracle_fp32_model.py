@@ -10,6 +10,7 @@ import pytest
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import fp32_model as F  # noqa: E402  (tests/fp32_model.py)
+import kernel_arith as K  # noqa: E402
 
 f32, f64 = np.float32, np.float64
 
@@ -42,7 +43,7 @@ def test_fma32_equals_rational_arithmetic_on_random_inputs():
     c = (rng.normal(size=n) * np.exp2(rng.integers(-140, 60, n))).astype(f32)
     c[:300] = (-(a[:300].astype(f64) * b[:300]).astype(f32))       # near-cancellation: the product's low bits decide
     a[300:400], b[300:400] = f32(2.0 ** -75), f32(1.5)              # results in fp32's subnormal range
-    got = F.fma32(a, b, c)
+    got = K.fma32(a, b, c)
     want = np.array([_fma_exact(*t) for t in zip(a, b, c)], f32)
     assert np.array_equal(got.view(np.int32), want.view(np.int32)), np.argwhere(got != want)[:5].ravel().tolist()
 
@@ -62,7 +63,7 @@ _DOUBLE_ROUNDING = [
 def test_fma32_rounds_once_where_fp64_rounds_twice(case):
     a, b, c = _DOUBLE_ROUNDING[case]
     want = _fma_exact(a, b, c)
-    assert F.fma32(a, b, c) == want
+    assert K.fma32(a, b, c) == want
     s = Fraction(float(a)) * Fraction(float(b)) + Fraction(float(c))
     mid = Fraction(float(f64(float(s))))                             # fl64(p + c) is an fp32 midpoint
     assert _rn32(mid) != want and mid != s
@@ -112,7 +113,7 @@ def test_rotate_volume_is_bit_identical_to_the_oracle_on_the_lattice(golden, ora
     rounds, where both restatements round the same way): the fp32 model and the oracle agree bit for bit, shared and
     per rotation."""
     vs = golden["shared_n3000_b3"]["vol_src"]
-    L = F.lattice_rotations()
+    L = K.lattice_rotations()
     ref = oracle.rotate_volume_np(vs[1], L)
     assert np.array_equal(F.rotate_volume(vs[1], L), ref)
     per = np.stack([vs[i % 3] for i in range(len(L))])
@@ -178,7 +179,7 @@ def test_target_feature_division_is_visible_to_bits_only(golden):
 
 def test_ulp_distance():
     one = f32(1.0)
-    assert F.ulp_distance(one, np.nextafter(one, f32(2.0))) == 1
-    assert F.ulp_distance(f32(0.0), f32(-0.0)) == 0
-    assert F.ulp_distance(np.nextafter(f32(0.0), f32(1.0)), np.nextafter(f32(0.0), f32(-1.0))) == 2
-    assert F.ulp_distance(f32(-1.0), f32(-1.0)) == 0
+    assert K.ulp_distance(one, np.nextafter(one, f32(2.0))) == 1
+    assert K.ulp_distance(f32(0.0), f32(-0.0)) == 0
+    assert K.ulp_distance(np.nextafter(f32(0.0), f32(1.0)), np.nextafter(f32(0.0), f32(-1.0))) == 2
+    assert K.ulp_distance(f32(-1.0), f32(-1.0)) == 0

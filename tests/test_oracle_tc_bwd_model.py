@@ -10,6 +10,7 @@ import pytest
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import tc_bwd_model as BM  # noqa: E402  (tests/tc_bwd_model.py)
+import kernel_arith as K  # noqa: E402
 import tc_model as M  # noqa: E402
 
 f32 = np.float32
@@ -113,7 +114,7 @@ def test_adjoint_path_choice(golden):
     cnt = BM.contributions(R)
     assert cnt.max() == 17 and 0 < (cnt > 16).mean() < 0.02
     assert np.bincount(cnt)[:9].sum() == 0                            # every rotation sends 9 or more to some voxel
-    assert BM.contributions(M.lattice_rotations()).max() == 8
+    assert BM.contributions(K.lattice_rotations()).max() == 8
     assert (BM.contributions(R[:300] * f32(0.35)) > 16).all()
     mixed = R[:300].copy()
     mixed[::5] *= f32(0.35)

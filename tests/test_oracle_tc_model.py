@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+import kernel_arith as K  # noqa: E402  (tests/kernel_arith.py)
 import tc_model as M  # noqa: E402  (tests/tc_model.py)
 
 f16, f32, f64 = np.float16, np.float32, np.float64
@@ -37,16 +38,17 @@ def test_fp32_gather_equals_rotate_volume_np(golden, oracle):
     """Bit-identical on lattice rotations (every weight is 0 or 1 up to the two base coordinates ATen rounds), within
     a few fp32 ulps of the volume's largest value otherwise (the kernel's FMAs against the oracle's rounded sums)."""
     vs = golden["shared_n3000_b3"]["vol_src"][1]
-    L = M.lattice_rotations()
-    assert np.array_equal(M.gather_f32(vs, L), oracle.rotate_volume_np(vs, L).reshape(len(L), 16, 512))
+    L = K.lattice_rotations()
+    assert np.array_equal(K.gather32(vs, L, parity="h", coords="tc"),
+                          oracle.rotate_volume_np(vs, L).reshape(len(L), 16, 512))
     R = golden["shared_n3000_b3"]["R"][:300]
-    got = M.gather_f32(vs, R).astype(f64)
+    got = K.gather32(vs, R, parity="h", coords="tc").astype(f64)
     ref = oracle.rotate_volume_np(vs, R).reshape(len(R), 16, 512)
     assert np.abs(got - ref).max() <= 8 * np.finfo(f32).eps * np.abs(vs).max()
     # and the 16-bit gather lies within fp16 interpolation error of the exact resampling
-    vh = M.rn16(vs * f32(1024.0))
+    vh = K.rn16(vs * f32(1024.0))
     got16 = M.gather_f16(vh, R).astype(f64) / 1024.0
-    assert np.abs(got16 - M.gather_f64(vs, R)).max() <= 8 * 2.0 ** -11 * np.abs(vs).max()
+    assert np.abs(got16 - K.gather64(vs, R)).max() <= 8 * 2.0 ** -11 * np.abs(vs).max()
 
 
 # ---- helpers --------------------------------------------------------------------------------------------------------
@@ -65,19 +67,19 @@ def test_rn16_matches_ieee_half():
         -65520.0: -np.inf,
     }
     for x, want in cases.items():
-        assert float(M.rn16(f64(x))) == want, x
+        assert float(K.rn16(f64(x))) == want, x
     x = np.random.default_rng(0).normal(size=20000) * np.exp2(np.random.default_rng(1).integers(-28, 17, 20000))
-    assert np.array_equal(M.rn16(x), x.astype(f16))
-    assert np.array_equal(M.rn16(x.astype(f32)), x.astype(f32).astype(f16))
+    assert np.array_equal(K.rn16(x), x.astype(f16))
+    assert np.array_equal(K.rn16(x.astype(f32)), x.astype(f32).astype(f16))
 
 
 def test_rz16_truncates():
     x = np.array([1.0 + 2.0 ** -11, -(1.0 + 2.0 ** -11), 1.0 + 2.0 ** -10 - 2.0 ** -30, 65520.0, 1e6, -1e6,
                   2.0 ** -24 * 1.9, 2.0 ** -25, 3.0])
     want = np.array([1.0, -1.0, 1.0, 65504.0, 65504.0, -65504.0, 2.0 ** -24, 0.0, 3.0])
-    assert np.array_equal(M.rz16(x).astype(f64), want)
+    assert np.array_equal(K.rz16(x).astype(f64), want)
     y = np.random.default_rng(2).normal(size=5000) * 100
-    r = M.rz16(y).astype(f64)
+    r = K.rz16(y).astype(f64)
     assert np.all(np.abs(r) <= np.abs(y)) and np.all(np.abs(y - r) < np.spacing(np.abs(r).astype(f16)).astype(f64))
 
 
@@ -85,14 +87,14 @@ def test_fma_is_fused():
     """Cases where a fused multiply-add and a rounded product followed by an add differ."""
     a = f32(1.0 + 2.0 ** -12)
     # a*a = 1 + 2^-11 + 2^-24: the rounded product loses 2^-24, the fused form keeps it
-    assert float(M.fma32(a, a, f32(-1.0))) == 2.0 ** -11 + 2.0 ** -24
+    assert float(K.fma32(a, a, f32(-1.0))) == 2.0 ** -11 + 2.0 ** -24
     assert float((a * a).astype(f32) - f32(1.0)) == 2.0 ** -11
     h = f16(1.0 + 2.0 ** -6)
     # h*h = 1 + 2^-5 + 2^-12: in fp16 the product rounds the 2^-12 away
-    assert float(M.fma16(h, h, f16(-1.0))) == 2.0 ** -5 + 2.0 ** -12
+    assert float(K.fma16(h, h, f16(-1.0))) == 2.0 ** -5 + 2.0 ** -12
     assert float(f16(h * h) - f16(1.0)) == 2.0 ** -5
     # a fused result that lands in fp16's subnormal range
-    assert float(M.fma16(f16(2.0 ** -12), f16(2.0 ** -12), f16(0.0))) == 2.0 ** -24
+    assert float(K.fma16(f16(2.0 ** -12), f16(2.0 ** -12), f16(0.0))) == 2.0 ** -24
 
 
 @pytest.mark.parametrize("k", [-20, -7, -1, 1, 5, 13])
