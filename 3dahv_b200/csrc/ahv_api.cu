@@ -106,13 +106,6 @@ bool screened(const VerifyWs& w, int vol_dtype, int math_mode, const float* scor
          N * sizeof(float) >= kScreenList * 10 * sizeof(float) && w.topk_bytes >= bytes_of<ScreenLists>(B);
 }
 
-// dist.shard_bounds: rank's contiguous share [lo, hi) of n items
-void shard_bounds(int64_t n, int rank, int world, int64_t* lo, int64_t* hi) {
-  const int64_t per = (n + world - 1) / world;
-  *lo = std::min(n, (int64_t)rank * per);
-  *hi = std::min(n, *lo + per);
-}
-
 // ---- chains: the device work of the entries, once their arguments have been checked -------------------------------
 // Each entry checks its arguments, then the device, then composes chains and launch_* functions; no entry calls
 // another (the host-buffer entries aside).  `pa` == nullptr or a group of one is one GPU.
@@ -179,7 +172,7 @@ int refine_gradient_chain(const Scored& p, const float* vol_tgt, int k, int step
   const ShardedRefineWs w(ws, B, N, k, pa ? pa->world : 1);
   const bool distinct = min_sep_deg > 0.0f;
   int64_t lo = 0, hi = N;
-  if (pa) shard_bounds(N, pa->rank, pa->world, &lo, &hi);
+  if (pa) peer::shard_bounds(N, pa->rank, pa->world, &lo, &hi);
   const int64_t n = hi - lo;
   const Scored slice = p.with_R(pa ? w.rs : p.R, p.r_per_pair, n);
   if (pa && n > 0)  // this rank's rotations, 16-byte aligned for the scorers (a shared set: one row)
@@ -214,7 +207,7 @@ int refine_gradient_chain(const Scored& p, const float* vol_tgt, int k, int step
   // empty slots (fewer than k distinct winners) are not ascended: R_all NaN, score_all -inf.  One GPU ascends every
   // slot (item_hi < 0), a rank its share, after which every ascended slot goes to every rank.
   int64_t ilo = 0, ihi = -1;
-  if (pa) shard_bounds((int64_t)B * k, pa->rank, pa->world, &ilo, &ihi);
+  if (pa) peer::shard_bounds((int64_t)B * k, pa->rank, pa->world, &ilo, &ihi);
   st = launch_gradient_ascent(p.with_R(first_R, true, k), w.tgt, steps, step_deg, R_all, score_all, s,
                               distinct ? first_idx : nullptr, ilo, ihi);
   if (st == AHV_OK && pa) st = launch_slot_gather(R_all, score_all, ilo, ihi, B, k, *pa, s);
@@ -918,20 +911,16 @@ AHV_API int ahv_peer_capacity_ex(const void* buf, int* max_pairs, int* max_k, in
 AHV_API int ahv_peer_close(void* ptr) { return (!ptr || cudaIpcCloseMemHandle(ptr) == cudaSuccess) ? AHV_OK : AHV_ECUDA; }
 
 namespace {
+// The group an entry is given: one GPU (world 1, rank 0), or peer::Args::valid.
 int make_peer_args(int rank, int world, void* const* peers, int peer_max_pairs, int peer_max_k, peer::Args* pa) {
-  if (world < 1 || world > peer::kMaxPeers || rank < 0 || rank >= world) return AHV_EINVAL;
   pa->rank = rank;
   pa->world = world;
   pa->cap_pairs = peer_max_pairs;
   pa->cap_k = peer_max_k;
-  if (world > 1) {
-    if (!peers || peer_max_pairs < 1 || !k_ok(peer_max_k)) return AHV_EINVAL;
-    for (int r = 0; r < world; ++r) {
-      if (!peers[r]) return AHV_EINVAL;
-      pa->bufs[r] = static_cast<unsigned char*>(peers[r]);
-    }
-  }
-  return AHV_OK;
+  if (world == 1) return rank == 0 ? AHV_OK : AHV_EINVAL;
+  if (peers && world <= peer::kMaxPeers)
+    for (int r = 0; r < world; ++r) pa->bufs[r] = static_cast<unsigned char*>(peers[r]);
+  return pa->valid() ? AHV_OK : AHV_EINVAL;
 }
 }  // namespace
 
@@ -964,7 +953,7 @@ AHV_API int ahv_verify_sharded(const void* vol_src, int vol_dtype, const float* 
   peer::Args pa;
   int st = make_peer_args(rank, world, peers, peer_max_pairs, peer_max_k, &pa);
   if (st != AHV_OK) return st;
-  if (world > 1 && (B > peer_max_pairs || k > peer_max_k)) return AHV_EINVAL;  // exchange buffer too small for this call
+  if (world > 1 && !pa.fits(B, k)) return AHV_EINVAL;
   st = check_device();
   if (st != AHV_OK) return st;
   if (world == 1 && N == 0) return AHV_EINVAL;
@@ -980,9 +969,9 @@ AHV_API int ahv_scores_exchange(const float* part, int B, int64_t N, float* scor
   peer::Args pa;
   int st = make_peer_args(rank, world, peers, peer_max_pairs, peer_max_k, &pa);
   if (st != AHV_OK) return st;
-  if (world < 2 || B > peer_max_pairs || !n_ok(peer_max_hyps) || N > peer_max_hyps) return AHV_EINVAL;
+  if (world < 2 || !n_ok(peer_max_hyps) || !pa.fits(B, 0, N, peer_max_hyps)) return AHV_EINVAL;
   int64_t lo, hi;
-  shard_bounds(N, rank, world, &lo, &hi);
+  peer::shard_bounds(N, rank, world, &lo, &hi);
   if (hi > lo && !part) return AHV_EINVAL;
   st = check_device();
   if (st != AHV_OK) return st;
@@ -1007,8 +996,8 @@ AHV_API int ahv_refine_gradient_sharded(const void* vol_src, int vol_dtype, cons
   peer::Args pa;
   int st = make_peer_args(rank, world, peers, peer_max_pairs, peer_max_k, &pa);
   if (st != AHV_OK) return st;
-  if (world > 1 && (B > peer_max_pairs || k > peer_max_k)) return AHV_EINVAL;  // the slot gather's entries
-  if (world > 1 && min_sep_deg > 0.0f && (!n_ok(peer_max_hyps) || N > peer_max_hyps)) return AHV_EINVAL;  // the score region
+  const int64_t hyps = min_sep_deg > 0.0f ? N : 0;  // the slot gather's entries; distinct winners: the score region too
+  if (world > 1 && (!pa.fits(B, k, hyps, peer_max_hyps) || (hyps > 0 && !n_ok(peer_max_hyps)))) return AHV_EINVAL;
   if (workspace_bytes < ShardedRefineWs(nullptr, B, N, k, world).total) return AHV_EWORKSPACE;
   st = check_device();
   if (st != AHV_OK) return st;

@@ -108,10 +108,14 @@ __device__ __forceinline__ Tap make_tap(const float* R, float x, float y, float 
 // (score, index) -> one ordered 64-bit key: larger key = higher score, ties -> lower index
 typedef unsigned long long u64;
 
+// score -> 32 bits whose unsigned order is the score order (-0 == +0): the high half of every key, and the score
+// comparison of the k = 1 peer merge
+__device__ __forceinline__ uint32_t score_bits(float score) {
+  const uint32_t u = __float_as_uint(score + 0.0f);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
 __device__ __forceinline__ u64 make_key(float score, uint32_t idx) {
-  uint32_t u = __float_as_uint(score + 0.0f);
-  u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-  return ((u64)u << 32) | (u64)(0xFFFFFFFFu - idx);
+  return ((u64)score_bits(score) << 32) | (u64)(0xFFFFFFFFu - idx);
 }
 __device__ __forceinline__ float key_score(u64 key) {
   uint32_t u = (uint32_t)(key >> 32);

@@ -262,10 +262,7 @@ static int make_finalize(float* best_val, int64_t* best_idx, float* R_best, int6
   fin->R_best = R_best;
   fin->idx_offset = idx_offset;
   if (pa && pa->world > 1) {
-    if (pa->world > peer::kMaxPeers || pa->rank < 0 || pa->rank >= pa->world || B > pa->cap_pairs || pa->cap_k < 1)
-      return AHV_EINVAL;
-    for (int r = 0; r < pa->world; ++r)
-      if (!pa->bufs[r]) return AHV_EINVAL;
+    if (!pa->fits(B, 1)) return AHV_EINVAL;
     fin->peers = *pa;
   }
   return AHV_OK;

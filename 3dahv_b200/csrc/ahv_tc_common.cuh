@@ -70,10 +70,8 @@ struct Finalize {
 __device__ __forceinline__ void peer_exchange_and_merge(const Finalize& fin, const u64* best_keys, const float* R,
                                                         int r_per_pair, int64_t N, int B, int lane) {
   const peer::Args& pa = fin.peers;
-  unsigned char* mine = pa.bufs[pa.rank];
-  uint32_t* hdr = reinterpret_cast<uint32_t*>(mine);
-  const uint32_t seq = *reinterpret_cast<volatile uint32_t*>(hdr) + 1u;
-  const int par = (int)(seq & 1u);
+  const unsigned char* mine = pa.bufs[pa.rank];
+  const peer::Step st = peer::open(pa);
   for (int b = lane; b < B; b += 32) {
     const u64 key = __ldcg(best_keys + b);
     const uint32_t n = key_index(key);
@@ -82,44 +80,34 @@ __device__ __forceinline__ void peer_exchange_and_merge(const Finalize& fin, con
 #pragma unroll
     for (int e = 0; e < 9; ++e) r9[e] = __ldg(src + e);
     const peer::Entry ent = peer::pack_entry((int64_t)n + fin.idx_offset, key_score(key), r9);
-    for (int p = 0; p < pa.world; ++p)  // NVLink peer stores (p == rank: local)
-      peer::store_entry(pa.bufs[p] + peer::entry_off(par, pa.rank, pa.cap_pairs, pa.cap_k, b, 0), ent);
+    peer::store_to_all(pa, st, pa.rank, b, 0, ent);
   }
-  __threadfence_system();  // entries before the flag, system scope
-  __syncwarp();
-  peer::publish_flags(pa, seq, par, lane);
-  const bool ok = __all_sync(0xffffffffu, peer::wait_flags(pa, seq, par, lane));
-  __threadfence_system();
+  const bool ok = peer::announce_and_wait(pa, st, lane);
   for (int b = lane; b < B; b += 32) {
-    float bv = 0.0f;
     uint32_t bo = 0;
     int64_t bi = -1;
-    uint4 bq0 = make_uint4(0, 0, 0, 0), bq1 = bq0, bq2 = bq0;
+    peer::Entry be = {};
     for (int r = 0; r < pa.world; ++r) {
-      const uint4* e = reinterpret_cast<const uint4*>(mine + peer::entry_off(par, r, pa.cap_pairs, pa.cap_k, b, 0));
-      const uint4 q0 = __ldcv(e);
+      const unsigned char* e = mine + peer::entry_off(st.par, r, pa.cap_pairs, pa.cap_k, b, 0);
+      const uint4 q0 = peer::load_head(e);
       const int64_t gi = peer::entry_index(q0);
-      const float v = __uint_as_float(q0.z);
-      const uint32_t o = peer::ordered_bits(v);
+      const uint32_t o = score_bits(peer::entry_score(q0));
       if (bi < 0 || o > bo || (o == bo && gi < bi)) {
-        bo = o; bv = v; bi = gi; bq0 = q0; bq1 = __ldcv(e + 1); bq2 = __ldcv(e + 2);
+        bo = o; bi = gi; be = peer::load_entry(e);
       }
     }
     const float nanv = __int_as_float(0x7fc00000);
-    fin.val[b] = ok ? bv : nanv;
+    fin.val[b] = ok ? peer::entry_score(be.q0) : nanv;
     fin.idx[b] = ok ? bi : -1;
     if (fin.R_best) {
       float o9[9];
-      peer::unpack_rotation(bq0, bq1, bq2, o9);
+      peer::unpack_rotation(be, o9);
 #pragma unroll
       for (int e = 0; e < 9; ++e) fin.R_best[b * 9 + e] = ok ? o9[e] : nanv;
     }
   }
   __syncwarp();
-  if (lane == 0) {
-    hdr[0] = seq;
-    if (!ok) hdr[1] = 1u;
-  }
+  if (lane == 0) peer::close(pa, st, ok);
 }
 
 struct Work {  // contiguous range of (pair, hypothesis) items of this CTA
